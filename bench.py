@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- the measurement contract of this repo.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference] [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[1]: Cornell box, the global_illumination example kernel
 (one sample per frame, seed = frameCount), 1920x1080, 64 frames kept as a running mean on the device,
@@ -16,12 +16,19 @@ GPU renders all of them (64*N spp).  Time = CUDA events on the stream the kernel
 --impl reference: the reference has no CPU implementation of this path and its OpenCL kernels cannot
 run here (no OpenCL ICD), so this arm times the CPU restatement of the same kernel (oracle/, "port")
 on all host cores, on a bounded sample of the same workload.
+
+--dump-outputs DIR: after the timed steps, the image the last timed step produced (what a caller of the timed
+path receives) is written as DIR/image.npy, float32 [H, W, 3] (--impl reference: the CPU port's frames of its last
+step, DIR/frames.npy [frames, H, W, 3]).  Output above 64 MB is written as a fixed, seeded sample of its pixels
+instead (DIR/image_sample.npy [n, 3] and their flat pixel indices DIR/image_sample_pixels.npy).  Inputs depend
+only on the arguments, so two builds of the project can be compared file by file.
 """
 import argparse
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import time
 
 import numpy as np
@@ -47,6 +54,23 @@ WORKLOADS = {
                              "synthetic 5M-triangle mesh, GI 4 bounces, 4K 256 spp"),
 }
 DEFAULT_WORKLOAD = "cornell_gi_1080p_64spp"
+DUMP_MAX_BYTES = 64 * 1000 * 1000
+
+
+def dump_outputs(out_dir, name, image):
+    """Writes the float32 [..., 3] image(s) of the last timed step as out_dir/<name>.npy, or, above DUMP_MAX_BYTES, a
+    fixed sample of their pixels (seed 0) as <name>_sample.npy [n, 3] with the flat pixel indices in
+    <name>_sample_pixels.npy (see --dump-outputs)."""
+    os.makedirs(out_dir, exist_ok=True)
+    image = np.ascontiguousarray(image, dtype=np.float32)
+    if image.nbytes <= DUMP_MAX_BYTES:
+        np.save(os.path.join(out_dir, name + ".npy"), image)
+        return
+    flat = image.reshape(-1, image.shape[-1])
+    n = (DUMP_MAX_BYTES - 4096) // (flat.shape[1] * 4 + 8)  # a pixel row + its float64 index; 4 KB for the headers
+    pixels = np.sort(np.random.default_rng(0).choice(len(flat), size=n, replace=False))
+    np.save(os.path.join(out_dir, name + "_sample.npy"), flat[pixels])
+    np.save(os.path.join(out_dir, name + "_sample_pixels.npy"), pixels.astype(np.float64))
 
 
 def load_scene(model, kind=0):
@@ -54,7 +78,7 @@ def load_scene(model, kind=0):
     from lens_trace_b200 import host
     if model.startswith("synth:"):
         n = int(model.split(":")[1])
-        path = "/tmp/lt_synth_%d_%d.obj" % (n, os.getpid())
+        path = os.path.join(tempfile.gettempdir(), "lt_synth_%d_%d.obj" % (n, os.getpid()))
         host.write_synthetic_scene(path, n, 0x5EED)
         sb = host.load_scene_buffers(path, kind)
         for p in (path, path[:-4] + ".mtl"):
@@ -120,8 +144,9 @@ class ClockSampler:
                 "samples": len(sm)}
 
 
-def cpu_oracle_rate(sb, kernel, w, h, depth, frame_list, threads=0):
-    """Mrays/s of the CPU restatement on `frame_list` full frames; returns (mrays_s, rays, seconds, cores)."""
+def cpu_oracle_rate(sb, kernel, w, h, depth, frame_list, threads=0, images=None):
+    """Mrays/s of the CPU restatement on `frame_list` full frames; returns (mrays_s, rays, seconds, cores).
+    The rendered frames are appended to `images` when it is a list."""
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import lt_oracle as O
     cores = os.cpu_count() or 1
@@ -129,9 +154,11 @@ def cpu_oracle_rate(sb, kernel, w, h, depth, frame_list, threads=0):
     for f in frame_list:
         cam = L.make_camera(0, 2.5, -50, 0.0, f)
         t0 = time.perf_counter()
-        _, st = O.render(kernel, sb, cam, w, h, max_ray_depth=depth if depth else 16, threads=threads, with_stats=True)
+        img, st = O.render(kernel, sb, cam, w, h, max_ray_depth=depth if depth else 16, threads=threads, with_stats=True)
         t += time.perf_counter() - t0
         rays += st.rays
+        if images is not None:
+            images.append(img)
     return rays / t / 1e6, rays, t, (threads if threads > 0 else cores)
 
 
@@ -176,12 +203,17 @@ def run_reference(args, rank, world):
     for i in range(max(0, args.warmup - 1)):
         cpu_oracle_rate(sb, kernel, w, h, depth, [i])
     rays, secs, port_secs, cores = 0, 0.0, 0.0, 1
+    frames_out = []
     for s in range(args.steps):
         fl = [s * per_step + k for k in range(per_step)]
-        _, r, t, cores = cpu_oracle_rate(sb, kernel, w, h, depth, fl)
+        frames_out.clear()
+        _, r, t, cores = cpu_oracle_rate(sb, kernel, w, h, depth, fl, images=frames_out)
         rays += r
         port_secs += t
         secs += cpu_reference_text_seconds(sb, kernel, w, h, depth, fl) if use_text else t
+    if args.dump_outputs and frames_out:
+        # the CPU port's frames of the last step, [per_step, H, W, 3]
+        dump_outputs(args.dump_outputs, "frames", np.stack(frames_out))
     value = rays / secs / 1e6
     sample = "%d of the %d frames per step at full %dx%d (frameCount = step*%d + k)" % (per_step, frames, w, h, per_step)
     line = {
@@ -458,7 +490,11 @@ def main():
     ap.add_argument("--no-cull", action="store_true", help="skip the secondary opt-in culled measurement")
     ap.add_argument("--no-lbvh", action="store_true", help="skip the secondary opt-in GPU-built LBVH measurement")
     ap.add_argument("--no-protocol", action="store_true", help="skip the reference-protocol (one render() per frame) timing")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the output of the last timed step to DIR as .npy files (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -576,6 +612,8 @@ def main():
     clocks = sampler.summary()
     launches_per_step = ctx.stats().kernel_launches
     result_image = acc.clone()  # what the last timed step left: the image every parity check below is about
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, "image", result_image.cpu().numpy())
 
     # The kernels timed in isolation, live, for the roofline: in the timed steps above consecutive batches of the
     # wavefront pipeline overlap on two streams (a trace kernel beside another batch's shade kernel), so a launch's

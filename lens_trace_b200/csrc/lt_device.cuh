@@ -190,10 +190,17 @@ __device__ __forceinline__ int lds32(unsigned addr) {
 
 // One 256-bit read-only load (LDG.E.ENL2.256.CONSTANT, sm_100): a 32-byte record costs one L1 request -- and, for
 // the divergent addresses of a traversal, one wavefront per distinct 128-byte line -- instead of two.
+// 256-bit loads need CUDA 12.9 or newer.  Plug-ins are compiled by whichever NVRTC the process has loaded (a PyTorch
+// built for CUDA 12.8 brings its own); with an older compiler the record is read as two 128-bit loads, same values.
 __device__ __forceinline__ void ldg256(const void* p, float4& a, float4& b) {
+#if __CUDACC_VER_MAJOR__ > 12 || (__CUDACC_VER_MAJOR__ == 12 && __CUDACC_VER_MINOR__ >= 9)
   asm volatile("ld.global.nc.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
                : "=f"(a.x), "=f"(a.y), "=f"(a.z), "=f"(a.w), "=f"(b.x), "=f"(b.y), "=f"(b.z), "=f"(b.w)
                : "l"(p));
+#else
+  asm volatile("ld.global.nc.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(a.x), "=f"(a.y), "=f"(a.z), "=f"(a.w) : "l"(p));
+  asm volatile("ld.global.nc.v4.f32 {%0,%1,%2,%3}, [%4+16];" : "=f"(b.x), "=f"(b.y), "=f"(b.z), "=f"(b.w) : "l"(p));
+#endif
 }
 
 // one inner-node step; requires t.cur >= 0

@@ -2,8 +2,12 @@
 Model / AccelerationStructureExplicit / RendererCUDA compiled from its sources (oracle/build_ref.sh);
 RendererCUDA NVRTC-compiles its basic.cu exactly as shipped.  Identical in-memory buffers go to the
 reference, to the new CUDA path and to the CPU oracle (the reference builder is nondeterministic, so
-buffers are never compared across builders)."""
+buffers are never compared across builders).
+
+Without the reference's sources the live tests skip; the stored outputs of the reference's CUDA backend
+(tests/golden/ref_cuda_*.npz, see tests/golden/README.md) keep the new CUDA path compared with it."""
 import ctypes as C
+import glob
 import os
 
 import numpy as np
@@ -107,6 +111,27 @@ def test_colour_and_hit_records_against_the_reference_cuda_backend(ref, ctx, nam
         util.assert_bit_equal(tuv[..., 0][ref_hit], a[..., 1][ref_hit], "t")
         util.assert_bit_equal(tuv[..., 1][ref_hit], a[..., 2][ref_hit], "u")
         util.assert_bit_equal(tuv[..., 2][ref_hit], b[..., 1][ref_hit], "v")
+    sc.release()
+
+
+@pytest.mark.parametrize("path", sorted(glob.glob(os.path.join(util.GOLDEN, "ref_cuda_*.npz"))),
+                         ids=lambda p: os.path.basename(p)[9:-4])
+def test_colour_and_hit_records_against_the_reference_golden(ctx, path):
+    """The reference's CUDA backend output stored with the buffers its builder made: the new CUDA path renders
+    the same picture and finds the same primary hits, bit for bit."""
+    z = np.load(path)
+    sb = L.SceneBuffers(z["nodes"], z["prims"], z["materials"], z["lights"])
+    cam = z["camera"].view(L.CAMERA)
+    w, h = int(z["width"]), int(z["height"])
+    sc = ctx.upload(sb)
+    mine = ctx.render(sc, cam, capi.make_params(L.KERNEL_BASIC_CU, w, h))
+    util.assert_bit_equal(mine, z["color"], os.path.basename(path) + ": new CUDA path vs reference CUDA backend")
+    if "ids" in z:
+        ids, hit, tuv = ctx.primary_hits(sc, cam, L.KERNEL_BASIC_CU, w, h)
+        m = z["hit"] == 1
+        np.testing.assert_array_equal(hit, z["hit"])
+        np.testing.assert_array_equal(ids[m], z["ids"][m])
+        util.assert_bit_equal(tuv[m], z["tuv"][m], os.path.basename(path) + " t,u,v")
     sc.release()
 
 

@@ -103,6 +103,17 @@ def test_cornell_box_loads_like_the_reference():
             assert sbx.materials["emission"][sbx.prims["mat"][p]].max() > 0
 
 
+@pytest.mark.parametrize("name", ["green_wall", "cornell_box", "cornell_box_lens"])
+def test_model_loader_matches_the_reference_loader_golden(name):
+    """This repo's OBJ/MTL reader on resources/models vs the triangles and materials the reference's loader made
+    (stored in tests/golden/ref_cuda_*.npz): the same primitives, in the reference builder's order or not."""
+    z = np.load(os.path.join(util.GOLDEN, "ref_cuda_%s_yaw000.npz" % name))
+    sb = util.scene(name)
+    key = lambda p: p.tobytes()
+    assert sorted(map(key, sb.prims)) == sorted(map(key, z["prims"]))
+    assert sb.materials.tobytes() == z["materials"].tobytes()
+
+
 def test_quad_split_rule(tmp_path):
     # shorter diagonal; a tie takes [0,1,3],[1,2,3] (tiny_obj_loader.h:1447-1487)
     obj = tmp_path / "q.obj"
