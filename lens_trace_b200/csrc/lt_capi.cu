@@ -139,10 +139,9 @@ extern "C" int lt_ctx_create(int device_ordinal, lt_ctx** out_ctx) {
   if (e2 == cudaSuccess) e2 = cudaEventCreate(&ctx->ev1);
   if (e2 == cudaSuccess) e2 = cudaMalloc(&ctx->dCounters, sizeof(LtCounters));
   if (e2 == cudaSuccess) e2 = cudaMalloc(&ctx->dWork, 256);
-  for (int k = 1; k < LT_WF_MAX_STREAMS; k++)
-    if (e2 == cudaSuccess) e2 = cudaStreamCreateWithFlags(&ctx->wfAux.extra[k], cudaStreamNonBlocking);
+  if (e2 == cudaSuccess) e2 = cudaStreamCreateWithFlags(&ctx->wfAux.extra, cudaStreamNonBlocking);
   if (e2 == cudaSuccess) e2 = cudaEventCreateWithFlags(&ctx->wfAux.fork, cudaEventDisableTiming);
-  for (int k = 0; k < LT_WF_MAX_STREAMS; k++)
+  for (int k = 0; k < 2; k++)
     if (e2 == cudaSuccess) e2 = cudaEventCreateWithFlags(&ctx->wfAux.order[k], cudaEventDisableTiming);
   if (e2 != cudaSuccess) {
     std::string m = std::string("lt_ctx_create: ") + cudaGetErrorString(e2);
@@ -175,14 +174,13 @@ extern "C" void lt_ctx_destroy(lt_ctx* ctx) {
   for (cudaEvent_t e : ctx->traceEvents) cudaEventDestroy(e);
   if (ctx->ev0) cudaEventDestroy(ctx->ev0);
   if (ctx->ev1) cudaEventDestroy(ctx->ev1);
-  for (int k = 1; k < LT_WF_MAX_STREAMS; k++)
-    if (ctx->wfAux.extra[k]) {
-      cudaStreamSynchronize(ctx->wfAux.extra[k]);
-      cudaStreamDestroy(ctx->wfAux.extra[k]);
-    }
+  if (ctx->wfAux.extra) {
+    cudaStreamSynchronize(ctx->wfAux.extra);
+    cudaStreamDestroy(ctx->wfAux.extra);
+  }
   if (ctx->wfAux.fork) cudaEventDestroy(ctx->wfAux.fork);
-  for (int k = 0; k < LT_WF_MAX_STREAMS; k++)
-    if (ctx->wfAux.order[k]) cudaEventDestroy(ctx->wfAux.order[k]);
+  for (cudaEvent_t e : ctx->wfAux.order)
+    if (e) cudaEventDestroy(e);
   if (ctx->ownStream) cudaStreamDestroy(ctx->ownStream);
   delete ctx;
 }
@@ -351,15 +349,11 @@ static int finish_scene(lt_ctx* ctx, lt_scene* s, int nNodes, int nPrims, int nM
     }
   }
   // large trees: the threaded copies are built on the device and used by coherent-ray launches only (lt_kernels.cu:
-  // scene_for_flags); skipped when they would not fit the budget (LT_THREADED_COHERENT_MAX_BYTES, default 4 GB)
+  // scene_for_flags); skipped when they would not fit the budget (4 GB and an eighth of the device)
   if (e == cudaSuccess && nNodes > lt_threaded_max_nodes() && nNodes > 1) {
-    static long long budget = -1;
-    if (budget < 0) {
-      const char* env = getenv("LT_THREADED_COHERENT_MAX_BYTES");
-      budget = env ? atoll(env) : (4ll << 30);
-    }
+    const size_t kBudget = 4ull << 30;
     const size_t bytes = sizeof(LtThreadNode) * 8 * (size_t)nNodes;
-    if ((long long)bytes <= budget && bytes <= ctx->totalMem / 8 && (long long)nNodes * 8 < 0x7fffffffll) {
+    if (bytes <= kBudget && bytes <= ctx->totalMem / 8 && (long long)nNodes * 8 < 0x7fffffffll) {
       if (cudaMalloc(&s->dThreadBig, bytes) == cudaSuccess) {
         lt_launch_build_threaded(s->dNodes, nNodes, s->dThreadBig, st);
         A(cudaGetLastError());
@@ -574,39 +568,6 @@ static int check_params(lt_ctx* ctx, const lt_scene* scene, const void* camera28
   L->accumMode = p->accum_mode;
   L->accumWeight = p->accum_weight;
   L->flags = p->flags;
-  {
-    // tuning knob (not part of the ABI): lanes below which a warp regenerates rays
-    static int threshold = -1;
-    if (threshold < 0) {
-      const char* e = getenv("LT_REFILL_THRESHOLD");
-      threshold = e ? atoi(e) : 4;
-      if (threshold < 1) threshold = 1;
-      if (threshold > 32) threshold = 32;
-    }
-    L->refillThreshold = threshold;
-    static int bAny = -1, bClosest = -1;
-    if (bAny < 0) {
-      const char* e = getenv("LT_BATCH_ANYHIT");
-      bAny = e ? atoi(e) : 16;
-      e = getenv("LT_BATCH_CLOSEST");
-      bClosest = e ? atoi(e) : 16;
-      bAny = bAny < 1 ? 1 : (bAny > 16 ? 16 : bAny);
-      bClosest = bClosest < 0 ? 0 : (bClosest > 16 ? 16 : bClosest);  // 0 selects the pipelined form in k_path
-    }
-    L->batchAnyHit = bAny;
-    L->batchClosest = bClosest;
-    static int iterNodes = -1, iterTris = -1;
-    if (iterNodes < 0) {
-      const char* e = getenv("LT_ITER_NODE_STEPS");
-      iterNodes = e ? atoi(e) : 8;
-      e = getenv("LT_ITER_TRI_TESTS");
-      iterTris = e ? atoi(e) : 3;
-      if (iterNodes < 1) iterNodes = 1;
-      if (iterTris < 1) iterTris = 1;
-    }
-    L->iterNodeSteps = iterNodes;
-    L->iterTriTests = iterTris;
-  }
   memcpy(&L->cam, camera28, sizeof(RefCamera));
   return LT_OK;
 }
@@ -633,13 +594,9 @@ static int render_common(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, float*
   int batchFrames = 1;
   if (L.kernel >= 3 && !(L.flags & LT_FLAG_MEGAKERNEL)) {
     long long pixels = (long long)L.width * L.height;
-    static long long minPaths = -1, maxPaths = -1;
-    if (minPaths < 0) {
-      const char* e = getenv("LT_WAVEFRONT_MIN_PATHS");
-      minPaths = e ? atoll(e) : (1ll << 23);
-      e = getenv("LT_WAVEFRONT_MAX_PATHS");
-      maxPaths = e ? atoll(e) : (1ll << 26);  // paths in flight, all overlapped batches together (~200 B each)
-    }
+    const long long minPaths = 1ll << 23;
+    // paths in flight, both overlapped batches together (~200 B each); a queue entry carries its path id in 25 bits
+    const long long maxPaths = 1ll << 26;
     // measured (tools/compare_pipelines.py): the wavefront wins once ~8M paths are in flight per batch; below
     // that, and for the two-ray lighting kernels on small scenes, its per-round launches and state traffic lose
     bool isGI = (L.kernel == 5 || L.kernel == 6);
@@ -665,26 +622,14 @@ static int render_common(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, float*
       long long cap = maxPaths;
       long long memCap = (long long)(ctx->totalMem / 8) / 200;  // at most 1/8 of the device for the workspace
       if (cap > memCap) cap = memCap;
-      if (cap > (1ll << 26)) cap = 1ll << 26;  // two batches; a queue entry carries its path id in 25 bits
       batchFrames = (int)(cap / pixels);
       if (batchFrames < 1) batchFrames = 1;
       if (batchFrames > L.frames) batchFrames = L.frames;
-      // consecutive batches overlap on LT_WF_OVERLAP (default 2) streams (trace of one beside shade of another): smaller batches,
-      // one workspace each -- same memory.  LT_FLAG_SERIAL / LT_WF_OVERLAP=1: one stream, kernels run one at a time.
-      static int overlapEnv = -1;
-      if (overlapEnv < 0) {
-        const char* e = getenv("LT_WF_OVERLAP");
-        overlapEnv = e ? atoi(e) : 2;  // batches in flight
-      }
-      overlapBatches = overlapEnv >= 2 && !(L.flags & (LT_FLAG_SERIAL | LT_FLAG_STATS)) && L.frames >= 2;
-      int nStreams = 1;
-      if (overlapBatches) {
-        nStreams = overlapEnv > LT_WF_MAX_STREAMS ? LT_WF_MAX_STREAMS : overlapEnv;
-        if (nStreams > L.frames) nStreams = L.frames;
-        if (batchFrames >= nStreams) batchFrames = (batchFrames + nStreams - 1) / nStreams;
-        else batchFrames = 1;
-        ctx->wfAux.streams = nStreams;
-      }
+      // two consecutive batches overlap on two streams (trace of one beside shade of the other): half-size batches,
+      // one workspace each -- same memory.  LT_FLAG_SERIAL: one stream, kernels run one at a time.
+      overlapBatches = !(L.flags & (LT_FLAG_SERIAL | LT_FLAG_STATS)) && L.frames >= 2;
+      const int nStreams = overlapBatches ? 2 : 1;
+      batchFrames = (batchFrames + nStreams - 1) / nStreams;
       {  // a queue entry carries its path id in 25 bits: at most 2^25 paths per batch
         long long perBatch = (1ll << 25) / pixels;
         if (perBatch < 1) perBatch = 1;
@@ -806,30 +751,22 @@ int lt_internal_download(lt_ctx* ctx, float* host_out, const float* dSrc, size_t
   memset(&attr, 0, sizeof attr);
   const bool pinned = cudaPointerGetAttributes(&attr, host_out) == cudaSuccess && attr.type == cudaMemoryTypeHost;
   cudaGetLastError();
-  static int threadsEnv = -1, minBytes = -1;
-  if (threadsEnv < 0) {
-    const char* e = getenv("LT_DOWNLOAD_THREADS");
-    // measured, 24.9 MB frame into a malloc'ed buffer: 2 threads 1.49 ms, 4: 0.93 ms, 8: 0.76 ms per render() call
-    unsigned hw = std::thread::hardware_concurrency();
-    threadsEnv = e ? atoi(e) : (hw >= 16 ? 8 : (hw >= 8 ? 4 : 2));
-    e = getenv("LT_DOWNLOAD_STAGED_MIN_BYTES");
-    minBytes = e ? atoi(e) : (1 << 20);
-  }
-  if (pinned || threadsEnv <= 0 || bytes < (size_t)minBytes) {
+  const size_t kStagedMinBytes = 1u << 20;  // smaller frames: one plain copy
+  if (pinned || bytes < kStagedMinBytes) {
     CK(cudaMemcpyAsync(host_out, dSrc, bytes, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     return LT_OK;
   }
-  static size_t kChunk = 0;  // staging granularity (LT_DOWNLOAD_CHUNK_KB)
-  if (kChunk == 0) {
-    const char* e = getenv("LT_DOWNLOAD_CHUNK_KB");
-    long kb = e ? atol(e) : 1024;  // measured 256 KB .. 2 MB with 8 .. 16 copier threads: 1 MB and 8 threads are best (0.68 ms per 1080p call)
-    if (kb < 64) kb = 64;
-    if (kb > 65536) kb = 65536;
-    kChunk = (size_t)kb << 10;
-  }
+  // staging granularity; measured 256 KB .. 2 MB with 8 .. 16 copier threads: 1 MB and 8 threads are best (0.68 ms per 1080p call)
+  const size_t kChunk = 1u << 20;
   const size_t kMaxStage = 256u << 20;
-  if (!ctx->copyPool) ctx->copyPool = new LtCopyPool(threadsEnv - 1);
+  if (!ctx->copyPool) {
+    // threads copying (this one included); measured, 24.9 MB frame into a malloc'ed buffer: 2 threads 1.49 ms,
+    // 4: 0.93 ms, 8: 0.76 ms per render() call
+    const unsigned hw = std::thread::hardware_concurrency();
+    const int threads = hw >= 16 ? 8 : (hw >= 8 ? 4 : 2);
+    ctx->copyPool = new LtCopyPool(threads - 1);
+  }
   if (ctx->stageBytes < (bytes < kMaxStage ? bytes : kMaxStage)) {
     if (ctx->stage) cudaFreeHost(ctx->stage);
     ctx->stage = nullptr;

@@ -129,7 +129,7 @@ struct Trav {
   int sp;
   int ignore;        // intersectIgnorePrimitiveIndex's primitive, < 0 = none
   bool anyHit;
-  int qHead, qTail;  // FIFO of reached-but-untested leaves (trav_iter), entries in the shared-memory list
+  int qHead, qTail;  // FIFO of reached-but-untested leaves (trav_iter_lean / trav_iter_threaded), shared-memory list
   Hit h;
 };
 
@@ -295,56 +295,18 @@ __device__ __forceinline__ bool trav_test(Trav& t, const LtSceneDev& sc, const i
   return false;
 }
 
-// Software-pipelined form for the persistent loops: because traversal never waits for triangle
-// results, one iteration advances the tree walk by up to `nodeSteps` box-pair tests (recording reached
-// leaves in a FIFO, in order) AND tests up to `triTests` recorded triangles (oldest first).  Within a
-// warp both halves of the iteration are populated by most lanes, whatever the phase of their rays.
-// Returns true when the ray is finished (tree exhausted and FIFO empty, or any-hit ray found a hit).
-template <bool STATS>
-__device__ __forceinline__ bool trav_iter(Trav& t, const LtSceneDev& sc, int* __restrict__ stk,
-                                          int* __restrict__ list, float epsThr, int nodeSteps, int triTests,
-                                          LtCounters& cnt) {
-  // a box-pair test, then record every leaf it (and the pops behind it) expose: cheap, and it keeps
-  // the lanes of a warp on the same instruction stream inside the loop
-  for (int steps = 0; steps < nodeSteps; steps++) {
-    if (t.cur >= 0) trav_node_step<STATS>(t, sc, stk, cnt);
-    // record the leaves this exposed (at most the near leaf, the far leaf and one popped leaf per
-    // step; anything beyond waits for the next step) -- straight-line code, no per-lane loop
-#pragma unroll
-    for (int k = 0; k < 3; k++) {
-      bool leaf = t.cur < 0 && t.cur != LT_DONE && t.qTail - t.qHead < LT_MAX_BATCH;
-      if (leaf) {
-        int prim = ~t.cur;
-        if (prim != t.ignore) {
-          list[(t.qTail & (LT_MAX_BATCH - 1)) * LT_THREAD_STRIDE] = prim;
-          t.qTail++;
-        }
-        t.cur = trav_pop(t, stk);
-      }
-    }
-    if (t.cur == LT_DONE || t.qTail - t.qHead >= LT_MAX_BATCH) break;
-  }
-  for (int k = 0; k < triTests && t.qHead != t.qTail; k++) {
-    int prim = list[(t.qHead & (LT_MAX_BATCH - 1)) * LT_THREAD_STRIDE];
-    t.qHead++;
-    if (STATS) cnt.triTests++;
-    if (tri_test(sc.tris, prim, t.r, epsThr, t.h)) {
-      t.h.prim = prim;
-      t.h.hit = 1;
-      if (t.anyHit) {
-        t.cur = LT_DONE;
-        t.qHead = t.qTail;
-      }
-    }
-  }
-  return t.cur == LT_DONE && t.qHead == t.qTail;
-}
-
-// ---- lean form of trav_iter for the persistent queue-fed kernel ---------------------------------
-// Same semantics; written for instruction count: shared memory is addressed through 32-bit shared
-// addresses (no generic-pointer conversion per access), the two children of a node are classified once
-// and a hit leaf child is recorded in the FIFO inside the node step itself (no pop/drain round trip);
-// only a leaf that had to wait on the stack behind an inner sibling is recorded after being popped.
+// ---- software-pipelined traversal for the persistent loops (k_flat_stream, k_wf_trace) ----------
+// Because traversal never waits for triangle results, one iteration advances the tree walk by up to
+// `nodeSteps` box-pair tests (recording reached leaves in a FIFO, in order) AND tests up to `triTests`
+// recorded triangles (oldest first).  Within a warp both halves of the iteration are populated by most
+// lanes, whatever the phase of their rays.  Returns true when the ray is finished (tree exhausted and
+// FIFO empty, or any-hit ray found a hit).  Written for instruction count: shared memory is addressed
+// through 32-bit shared addresses (no generic-pointer conversion per access), the two children of a node
+// are classified once and a hit leaf child is recorded in the FIFO inside the node step itself (no
+// pop/drain round trip); only a leaf that had to wait on the stack behind an inner sibling is recorded
+// after being popped.
+constexpr int kLeanNodeSteps = 8;  // box-pair tests per iteration
+constexpr int kLeanTriTests = 3;   // triangle tests per iteration
 template <bool STATS>
 __device__ __forceinline__ bool trav_iter_lean(Trav& t, const LtSceneDev& sc, unsigned stkAddr, unsigned fifoAddr,
                                                float epsThr, int nodeSteps, int triTests, LtCounters& cnt) {
@@ -491,6 +453,10 @@ __device__ __forceinline__ void trav_threaded_nodes(Trav& t, const LtThreadNode*
   }
 }
 
+// iteration shape of the persistent loops (k_path, k_wf_trace) on the threaded tree: single-box steps, so twice the
+// steps of kLeanNodeSteps
+constexpr int kThreadedNodeSteps = 2 * kLeanNodeSteps;
+constexpr int kThreadedTriTests = kLeanTriTests;
 __device__ __forceinline__ bool trav_iter_threaded(Trav& t, const LtThreadNode* __restrict__ tn,
                                                    const LtTri* __restrict__ tris, unsigned fifoAddr, float epsThr,
                                                    int nodeSteps, int triTests) {

@@ -13,11 +13,6 @@ struct LtLaunch {
   int accumMode;
   float accumWeight;
   int flags;
-  int refillThreshold;  // k_path: leave the traversal loop when fewer lanes than this still have a ray
-  int batchAnyHit;      // k_path: leaves recorded before a shadow ray tests them (early-out granularity)
-  int batchClosest;     // k_path: leaves recorded before a closest-hit ray tests them
-  int iterNodeSteps;    // trav_iter: box-pair tests per iteration of a persistent loop
-  int iterTriTests;     // trav_iter: triangle tests per iteration
   // Row window of a tile split (multi-GPU): this launch renders `height` rows of an image of `fullHeight` rows;
   // local row j is image row ((j / rowBlock) * rowStride + rowPhase) * rowBlock + j % rowBlock (blocks of rowBlock
   // rows dealt round-robin to rowStride devices).  rowStride <= 1: the whole image (fullHeight == height).

@@ -32,15 +32,13 @@ size_t lt_wf_workspace_bytes_padded(long long nPaths);
 size_t lt_wf_primary_hits_bytes(long long pixels);  // per-launch primary hit records, kept behind the batch workspaces
 // traceEvents: optional pool of 2*maxTraceLaunches events; when given, every traversal launch is bracketed by a
 // pair of events and *traceLaunches receives the number of pairs recorded
-// aux: extra streams + events (fork, one batch-order event per stream) for overlapping consecutive batches (the
-// L1-bound trace kernel of one batch runs beside the DRAM-bound shade kernel of another and fills the tail of the
-// persistent kernels); `workspace` then holds aux->streams
-// batch workspaces of lt_wf_workspace_bytes_padded(batchFrames * pixels) each.  aux == nullptr: one stream.
-#define LT_WF_MAX_STREAMS 4
+// aux: a second stream + events (fork, one batch-order event per stream) for overlapping consecutive batches (the
+// L1-bound trace kernel of one batch runs beside the DRAM-bound shade kernel of the other and fills the tail of the
+// persistent kernels); `workspace` then holds two batch workspaces of
+// lt_wf_workspace_bytes_padded(batchFrames * pixels) each.  aux == nullptr: one stream.
 struct LtWfAux {
-  int streams;                              // batches in flight (2..LT_WF_MAX_STREAMS), one stream each
-  cudaStream_t extra[LT_WF_MAX_STREAMS];    // [0] unused: side 0 runs on the caller's stream
-  cudaEvent_t fork, order[LT_WF_MAX_STREAMS];
+  cudaStream_t extra;  // odd batches; even batches run on the caller's stream
+  cudaEvent_t fork, order[2];
 };
 // pairKinds: optional, one LT_TIMED_* per recorded pair; when given, the shade / primary-shade / accumulate launches
 // are bracketed as well (per-kernel times of a serialised step)

@@ -107,7 +107,7 @@ __global__ void __launch_bounds__(LT_BLOCK) k_flat_stream(LtSceneDev sc, LtLaunc
     int ignore = -1;
     for (int stage = 0; stage < 3; stage++) {  // 0 camera ray, 1 and 2 the rays through a lens (basic.cu:245-298)
       trav_begin<false>(t, sc, ignore, tInit, false, cnt);
-      while (!trav_iter_lean<false>(t, sc, stkAddr, fifoAddr, epsThr, L.iterNodeSteps, L.iterTriTests, cnt)) {
+      while (!trav_iter_lean<false>(t, sc, stkAddr, fifoAddr, epsThr, kLeanNodeSteps, kLeanTriTests, cnt)) {
       }
       const Hit h = t.h;
       if (stage == 0) {
@@ -146,15 +146,17 @@ __global__ void __launch_bounds__(LT_BLOCK) k_flat_stream(LtSceneDev sc, LtLaunc
 //   S (shade/regenerate): lanes whose ray has finished consume the hit and produce their next ray
 //     (primary, shadow or extension); the hash-RNG draws, the expensive part, are one shared code
 //     site whatever the path stage;
-//   T (traverse): all lanes with an unfinished ray run the while-while traversal; the loop is left
-//     as soon as fewer than L.refillThreshold lanes are still traversing and some lane is waiting
-//     for a new ray, so long rays never hold the other 31 lanes idle.  Traversal state is resumable.
+//   T (traverse): all lanes with an unfinished ray run the traversal in its leaf-list form (whole
+//     batches of box tests, then the recorded triangles; the stackless form on a threaded tree); the
+//     loop is left as soon as fewer than kPathRefillLanes lanes are still traversing and some lane is
+//     waiting for a new ray, so long rays never hold the other 31 lanes idle.  Traversal state is
+//     resumable.
+constexpr int kPathRefillLanes = 4;
 template <bool STATS>
 __global__ void __launch_bounds__(LT_BLOCK) k_path(LtSceneDev sc, LtLaunch L, float* __restrict__ out,
                                                    LtCounters* gcnt) {
   LT_SMEM_POINTERS(sc)
   (void)tstk;  // the persistent megakernel does not cull (LT_FLAG_CULL selects the wavefront pipeline)
-  const unsigned stkAddr = (unsigned)__cvta_generic_to_shared(stk);
   const unsigned fifoAddr = (unsigned)__cvta_generic_to_shared(list);
   int px, py;
   bool alive = thread_pixel(L.width, L.height, px, py);
@@ -235,16 +237,14 @@ __global__ void __launch_bounds__(LT_BLOCK) k_path(LtSceneDev sc, LtLaunch L, fl
       unsigned active = __ballot_sync(0xffffffffu, traversing);
       if (active == 0u) break;
       bool waiting = __any_sync(0xffffffffu, alive && !traversing);
-      if (waiting && __popc(active) < L.refillThreshold) break;
+      if (waiting && __popc(active) < kPathRefillLanes) break;
       if (traversing) {
         if (threaded) {
-          traversing = !trav_iter_threaded(t, sc.tnodes, sc.tris, fifoAddr, pc.epsThr, 2 * L.iterNodeSteps, L.iterTriTests);
-        } else if (L.batchClosest > 0) {  // leaf-list form: whole batches of box tests, then the recorded triangles
-          int n = trav_collect<STATS>(t, sc, stk, list, t.anyHit ? L.batchAnyHit : L.batchClosest, cnt);
+          traversing = !trav_iter_threaded(t, sc.tnodes, sc.tris, fifoAddr, pc.epsThr, kThreadedNodeSteps, kThreadedTriTests);
+        } else {
+          int n = trav_collect<STATS>(t, sc, stk, list, LT_MAX_BATCH, cnt);
           trav_test<STATS>(t, sc, list, n, pc.epsThr, cnt);
           traversing = (t.cur != LT_DONE);
-        } else {  // software-pipelined form (same as the wavefront trace kernel)
-          traversing = !trav_iter_lean<STATS>(t, sc, stkAddr, fifoAddr, pc.epsThr, L.iterNodeSteps, L.iterTriTests, cnt);
         }
       }
     }

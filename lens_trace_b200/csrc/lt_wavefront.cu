@@ -18,6 +18,10 @@
 
 #define WF_BLOCK LT_BLOCK
 #define WF_CHUNK 128  // queue entries a warp claims per global atomic (measured 32..1024: 64-256 equal, 1024 -8 %)
+// idle lanes a warp waits for before it fetches new rays: lanes that start together walk the top of the tree
+// together and share its cache lines (measured: 8 is ~1 % faster than 1 on both the 83-node and the 2 M-node tree)
+#define WF_REFILL_LANES 8
+#define WF_THREADED_BLOCKS_PER_SM 8  // persistent trace blocks per SM on the threaded tree
 
 struct LtWfBuffers {
   float4* st;         // 64-byte record per path, two 32-byte sectors that are read and written independently:
@@ -286,10 +290,13 @@ __global__ void k_wf_reset(LtWfBuffers B) {
 // persistent trace: lanes pull queue entries through one warp-aggregated atomic per refill
 // THREADED: stackless traversal of the per-octant threaded tree (sc.tnodes, small scenes); shared memory then
 // holds only the leaf FIFO.  Same tests in the same order, hence the same hit records.
+// Exact variants: at most 56 registers, so that one block of the other batch's shade kernel (64 registers) fits on an
+// SM beside 8 trace blocks.  Left to itself ptxas gives the stack variant 64 registers (no spill instead of 4 bytes),
+// and the 1M-triangle GI step then takes 42.7 instead of 42.0-42.4 ms (B200, 1000 W power limit).
 template <bool STATS, bool THREADED>
-__global__ void __launch_bounds__(WF_BLOCK) k_wf_trace(LtSceneDev sc, LtLaunch L, LtWfBuffers B, int q,
-                                                       LtCounters* gcnt, const float4* __restrict__ rayO,
-                                                       const float4* __restrict__ rayD) {
+__global__ void __launch_bounds__(WF_BLOCK) __maxnreg__(STATS ? 64 : 56)
+    k_wf_trace(LtSceneDev sc, LtLaunch L, LtWfBuffers B, int q, LtCounters* gcnt, const float4* __restrict__ rayO,
+               const float4* __restrict__ rayD) {
   extern __shared__ int smemStack[];
   int* stk = smemStack + threadIdx.x;
   int* list = smemStack + (THREADED ? 0 : lt_stack_levels(sc) * LT_BLOCK) + threadIdx.x;
@@ -314,13 +321,13 @@ __global__ void __launch_bounds__(WF_BLOCK) k_wf_trace(LtSceneDev sc, LtLaunch L
   while (true) {
     bool has = entry >= 0;
     unsigned need = __ballot_sync(0xffffffffu, !has);
-    if (__popc(need) >= L.refillThreshold && !exhausted) {
+    if (__popc(need) >= WF_REFILL_LANES && !exhausted) {
       if (chunkNext >= chunkEnd) {
         int base = 0;
-        if (lane == 0u) base = atomicAdd(&B.counts[4], L.batchClosest);  // chunk size (host: LT_WF_CHUNK)
+        if (lane == 0u) base = atomicAdd(&B.counts[4], WF_CHUNK);
         base = __shfl_sync(0xffffffffu, base, 0);
         chunkNext = base;
-        chunkEnd = min(base + L.batchClosest, n);
+        chunkEnd = min(base + WF_CHUNK, n);
         if (base >= n) exhausted = true;
       }
       if (!exhausted) {
@@ -350,13 +357,13 @@ __global__ void __launch_bounds__(WF_BLOCK) k_wf_trace(LtSceneDev sc, LtLaunch L
     if (has) {
       bool finished;
       if (THREADED) {
-        finished = trav_iter_threaded(t, sc.tnodes, sc.tris, fifoAddr, epsThr, L.iterNodeSteps, L.iterTriTests);
+        finished = trav_iter_threaded(t, sc.tnodes, sc.tris, fifoAddr, epsThr, kThreadedNodeSteps, kThreadedTriTests);
       } else if (cull && !t.anyHit) {  // a round holds one kind of ray, so this does not split warps
-        for (int k = 0; k < 2 * L.iterNodeSteps && t.cur != LT_DONE; k++)
+        for (int k = 0; k < 2 * kLeanNodeSteps && t.cur != LT_DONE; k++)
           trav_step_cull<STATS>(t, sc, stk, tstk, epsThr, cnt);
         finished = t.cur == LT_DONE;
       } else {
-        finished = trav_iter_lean<STATS>(t, sc, stkAddr, fifoAddr, epsThr, L.iterNodeSteps, L.iterTriTests, cnt);
+        finished = trav_iter_lean<STATS>(t, sc, stkAddr, fifoAddr, epsThr, kLeanNodeSteps, kLeanTriTests, cnt);
       }
       if (finished) {
         B.hits[entry] = make_float4(t.h.t, t.h.u, t.h.v,
@@ -493,11 +500,6 @@ __global__ void __launch_bounds__(WF_BLOCK) k_wf_accumulate(LtLaunch L, LtWfBuff
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
-#include <stdlib.h>
-static int lt_env_int(const char* name, int dflt) {  // tuning knobs for experiments; defaults are the measured choice
-  const char* e = getenv(name);
-  return e ? atoi(e) : dflt;
-}
 #define LT_LAUNCH_FLAG_NO_THREADED 16  // == LT_FLAG_NO_THREADED (include/lens_trace_b200.h)
 
 size_t lt_wf_bytes_per_path() {
@@ -586,29 +588,18 @@ int lt_launch_render_wavefront(const LtSceneDev& scIn, const LtLaunch& L, float*
   // stack kernel, whose tests are the same ones)
   const bool threaded = sc.tnodes != nullptr;
   const size_t smemTrace = threaded ? (size_t)LT_MAX_BATCH * LT_BLOCK * sizeof(int) : smem;
-  LtLaunch Lt = L;  // iteration shape of the trace kernel: single-box steps when threaded
-  // idle lanes a warp waits for before it fetches new rays: lanes that start together walk the top of the tree
-  // together and share its cache lines (measured: 8 is ~1 % faster than 1 on both the 83-node and the 2 M-node tree)
-  Lt.refillThreshold = lt_env_int("LT_WF_REFILL_LANES", 8);
-  if (threaded) {
-    blocksPerSm = lt_env_int("LT_THREADED_BLOCKS_PER_SM", 8);
-    Lt.iterNodeSteps = lt_env_int("LT_THREADED_NODE_STEPS", 2 * L.iterNodeSteps);
-    Lt.iterTriTests = lt_env_int("LT_THREADED_TRI_TESTS", L.iterTriTests);
-  }
-  // Two batches in flight on two streams: the persistent trace kernel leaves room on every SM for blocks of the
-  // other batch's shade kernel (different bottlenecks: L1 data pipe vs DRAM).
+  if (threaded) blocksPerSm = WF_THREADED_BLOCKS_PER_SM;
+  // Two batches in flight on two streams: the trace kernel of one batch runs beside the shade kernel of the other
+  // (different bottlenecks: L1 data pipe vs DRAM).  Measured: reserving room on the SMs for the other batch's blocks
+  // (fewer persistent trace blocks) does not pay, nor do 3 or 4 batches in flight (profiles/r2u_overlap_sweep.txt).
   const bool overlap = aux != nullptr && L.frames > batchFrames;
-  const int nStreams = overlap ? aux->streams : 1;
-  if (overlap) {  // measured: reserving room for the other batch's blocks (fewer persistent blocks) does not pay
-    int cap = lt_env_int("LT_WF_OVERLAP_TRACE_BLOCKS_PER_SM", 8);
-    if (blocksPerSm > cap) blocksPerSm = cap;
-  }
+  const int nStreams = overlap ? 2 : 1;
   const int persistentBlocks = smCount * blocksPerSm;
   const size_t wsBytes = lt_wf_workspace_bytes_padded((long long)batchFrames * pixels);
   int preLaunches = 0;
   // primary hits once per pixel per launch (exact, uncounted pipelines); kept behind the batch workspaces
   LtWfPrimary P = {};
-  if (!stats && !(L.flags & 2) && lt_env_int("LT_WF_SHARED_PRIMARY", 1)) {
+  if (!stats && !(L.flags & 2)) {
     char* pb = (char*)workspace + (size_t)nStreams * wsBytes;  // 256-aligned: wsBytes is a multiple of 256
     auto take = [&](size_t bytes) {
       char* r = pb;
@@ -621,7 +612,7 @@ int lt_launch_render_wavefront(const LtSceneDev& scIn, const LtLaunch& L, float*
     while ((1ll << l) < pixels) l++;
     P.divS = 25 + l;
     P.divM = (unsigned long long)(((1ull << P.divS) + (unsigned long long)pixels - 1ull) / (unsigned long long)pixels);
-    const bool classify = samples == 1 && lt_env_int("LT_WF_ALIVE_LIST", 1);
+    const bool classify = samples == 1;
     if (classify) {
       P.alive = (int*)take(sizeof(int) * (size_t)pixels);
       P.aliveCount = (int*)take(256);
@@ -636,12 +627,12 @@ int lt_launch_render_wavefront(const LtSceneDev& scIn, const LtLaunch& L, float*
   float4* primaryHits = P.hits;
   if (overlap) {
     cudaEventRecord(aux->fork, stream);
-    for (int k = 1; k < nStreams; k++) cudaStreamWaitEvent(aux->extra[k], aux->fork, 0);
+    cudaStreamWaitEvent(aux->extra, aux->fork, 0);
   }
   int launches = preLaunches, batch = 0, lastSide = 0;
   for (int frame0 = 0; frame0 < L.frames; frame0 += batchFrames, batch++) {
-    const int side = overlap ? (batch % nStreams) : 0;
-    cudaStream_t st = side ? aux->extra[side] : stream;
+    const int side = overlap ? (batch & 1) : 0;
+    cudaStream_t st = side ? aux->extra : stream;
     int nf = L.frames - frame0 < batchFrames ? L.frames - frame0 : batchFrames;
     long long nPaths = (long long)nf * pixels;
     LtWfBuffers B = carve((char*)workspace + (size_t)side * wsBytes, (long long)batchFrames * pixels);
@@ -661,14 +652,9 @@ int lt_launch_render_wavefront(const LtSceneDev& scIn, const LtLaunch& L, float*
       int q = 0;
       for (int r = 1; r < rounds; r++) {
         mark(0, st);
-        LtLaunch Lq = Lb;  // iteration shape of the trace kernel
-        Lq.iterNodeSteps = Lt.iterNodeSteps;
-        Lq.iterTriTests = Lt.iterTriTests;
-        Lq.refillThreshold = Lt.refillThreshold;
-        Lq.batchClosest = lt_env_int("LT_WF_CHUNK", WF_CHUNK);  // k_path's field, reused: entries per work claim
-        if (stats) k_wf_trace<true, false><<<persistentBlocks, WF_BLOCK, smem, st>>>(sc, Lq, B, q, dCounters, B.rayO[q], B.rayD[q]);
-        else if (threaded) k_wf_trace<false, true><<<persistentBlocks, WF_BLOCK, smemTrace, st>>>(sc, Lq, B, q, nullptr, B.rayO[q], B.rayD[q]);
-        else k_wf_trace<false, false><<<persistentBlocks, WF_BLOCK, smem, st>>>(sc, Lq, B, q, nullptr, B.rayO[q], B.rayD[q]);
+        if (stats) k_wf_trace<true, false><<<persistentBlocks, WF_BLOCK, smem, st>>>(sc, Lb, B, q, dCounters, B.rayO[q], B.rayD[q]);
+        else if (threaded) k_wf_trace<false, true><<<persistentBlocks, WF_BLOCK, smemTrace, st>>>(sc, Lb, B, q, nullptr, B.rayO[q], B.rayD[q]);
+        else k_wf_trace<false, false><<<persistentBlocks, WF_BLOCK, smem, st>>>(sc, Lb, B, q, nullptr, B.rayO[q], B.rayD[q]);
         mark(1, st);
         mark(0, st, LT_TIMED_SHADE);
         if (q == 0) k_wf_shade<0><<<grid, WF_BLOCK, 0, st>>>(sc, Lb, B, pixels, 0, s, P);
@@ -680,7 +666,7 @@ int lt_launch_render_wavefront(const LtSceneDev& scIn, const LtLaunch& L, float*
       }
     }
     // the frame combiner is applied in frame order: this batch's accumulate follows the previous batch's
-    if (overlap && batch > 0) cudaStreamWaitEvent(st, aux->order[(side + nStreams - 1) % nStreams], 0);
+    if (overlap && batch > 0) cudaStreamWaitEvent(st, aux->order[1 - side], 0);
     mark(0, st, LT_TIMED_ACCUMULATE);
     k_wf_accumulate<<<(pixels + WF_BLOCK - 1) / WF_BLOCK, WF_BLOCK, 0, st>>>(L, B, dOut, pixels, frame0, nf, P.cls);
     mark(1, st, LT_TIMED_ACCUMULATE);

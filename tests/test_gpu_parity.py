@@ -216,30 +216,22 @@ def test_overlapped_batches_equal_one_stream(ctx, kernel, depth, frames):
 
 
 def test_shared_primary_hits_equal_per_frame_tracing(ctx):
-    """The wavefront pipeline traces the camera ray of a pixel once per launch and starts every frame's path from
-    that record (the ray is the same in every frame); LT_WF_SHARED_PRIMARY=0 traces it per frame as the
-    reference does."""
+    """The wavefront pipeline traces the camera ray of a pixel once per launch, starts every frame's path from that
+    record (the ray is the same in every frame) and gives paths only to the pixels whose camera ray hits a surface
+    (black / white pixels are constant).  Its stats launch traces the camera ray per frame and gives every pixel a
+    path, and the megakernel traces it per frame as the reference does: all three images are the same."""
     sb, sc = gpu_scene(ctx, "cornell_box_lens")
     cam = util.default_camera(0.01, 2)
-    p = capi.make_params(L.KERNEL_GI, 200, 150, max_ray_depth=3, frames=5, accum_mode=L.ACCUM_RUNNING_MEAN,
-                         flags=L.FLAG_WAVEFRONT)
-    ctx.accum_reset()
-    shared = ctx.render(sc, cam, p).copy()
-    os.environ["LT_WF_SHARED_PRIMARY"] = "0"
-    try:
+
+    def gi(flags):
         ctx.accum_reset()
-        per_frame = ctx.render(sc, cam, p).copy()
-    finally:
-        os.environ.pop("LT_WF_SHARED_PRIMARY")
-    util.assert_bit_equal(shared, per_frame, "shared vs per-frame primary hits")
-    # ... and gives paths only to the pixels whose camera ray hits a surface (black / white pixels are constant)
-    os.environ["LT_WF_ALIVE_LIST"] = "0"
-    try:
-        ctx.accum_reset()
-        all_pixels = ctx.render(sc, cam, p).copy()
-    finally:
-        os.environ.pop("LT_WF_ALIVE_LIST")
-    util.assert_bit_equal(shared, all_pixels, "alive-pixel list vs paths for every pixel")
+        return ctx.render(sc, cam, capi.make_params(L.KERNEL_GI, 200, 150, max_ray_depth=3, frames=5,
+                                                    accum_mode=L.ACCUM_RUNNING_MEAN, flags=flags)).copy()
+
+    shared = gi(L.FLAG_WAVEFRONT)
+    util.assert_bit_equal(shared, gi(L.FLAG_WAVEFRONT | L.FLAG_STATS),
+                          "shared primary hits + alive list vs per-frame tracing for every pixel (stats launch)")
+    util.assert_bit_equal(shared, gi(L.FLAG_MEGAKERNEL), "shared primary hits + alive list vs megakernel")
     lit = capi.make_params(L.KERNEL_ACCUMULATOR, 200, 150, frames=5, accum_mode=L.ACCUM_RUNNING_MEAN, flags=L.FLAG_WAVEFRONT)
     mega = capi.make_params(L.KERNEL_ACCUMULATOR, 200, 150, frames=5, accum_mode=L.ACCUM_RUNNING_MEAN, flags=L.FLAG_MEGAKERNEL)
     ctx.accum_reset()

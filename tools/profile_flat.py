@@ -29,7 +29,7 @@ def main():
         for _ in range(reps):
             ctx.render(scene, cam, p, want_output=False)
             ms.append(ctx.stats().kernel_ms)
-        knobs = " ".join("%s=%s" % (k, v) for k, v in sorted(os.environ.items()) if k.startswith(("LT_STREAM", "LT_ITER", "LT_BATCH", "LT_THREADED", "LT_PROFILE_FLAGS")))
+        knobs = " ".join("%s=%s" % (k, v) for k, v in sorted(os.environ.items()) if k.startswith(("LT_STREAM", "LT_THREADED", "LT_PROFILE_FLAGS")))
         print("%s kernel %d %dx%d [%s]: ms %s" % (model, kernel, w, h, knobs, " ".join("%.4f" % m for m in ms)), flush=True)
     if not os.environ.get("LT_PROFILE_NOREF"):
         ref = bench.reference_cuda_kernel_rate(sb, w, h)

@@ -1,8 +1,7 @@
-"""Times the wavefront pipeline with the stackless threaded traversal against the stack traversal, and sweeps the
-iteration shape of the threaded trace kernel (env knobs read at every launch by lt_wavefront.cu).
-    python tools/tune_threaded.py [sweep]
+"""Times the wavefront pipeline with the stackless threaded traversal against the stack traversal, and two
+overlapped batches against one stream (LT_FLAG_SERIAL); checks that the images are identical.
+    python tools/tune_threaded.py
 """
-import itertools
 import os
 import sys
 
@@ -25,7 +24,6 @@ def timed(ctx, sc, cam, p, n=4):
 
 
 def main():
-    sweep = len(sys.argv) > 1 and sys.argv[1] == "sweep"
     ctx = capi.Context(0)
     cam = L.make_camera(0, 2.5, -50)
     cases = [("cornell_box", L.KERNEL_GI, 1920, 1080, 64, 4), ("cornell_box", L.KERNEL_ACCUMULATOR, 1920, 1080, 64, 0),
@@ -53,20 +51,6 @@ def main():
         t2, tr2 = timed(ctx, sc, cam, ser)
         print("      one stream (LT_FLAG_SERIAL): threaded %.2f ms (trace %.2f)  identical=%s" % (
             t2, tr2, bool((c.view(np.uint32) == b.view(np.uint32)).all())), flush=True)
-        for blocks in (3, 4, 5, 6, 8):
-            os.environ["LT_WF_OVERLAP_TRACE_BLOCKS_PER_SM"] = str(blocks)
-            t, tr = timed(ctx, sc, cam, thr, n=3)
-            print("      overlap, trace blocks/SM %d: %.2f ms" % (blocks, t), flush=True)
-        os.environ.pop("LT_WF_OVERLAP_TRACE_BLOCKS_PER_SM")
-        if sweep and model == "cornell_box" and kernel == L.KERNEL_GI:
-            for steps, tris, blocks in itertools.product((8, 12, 16, 24), (2, 3, 4, 6), (6, 8, 12)):
-                os.environ["LT_THREADED_NODE_STEPS"] = str(steps)
-                os.environ["LT_THREADED_TRI_TESTS"] = str(tris)
-                os.environ["LT_THREADED_BLOCKS_PER_SM"] = str(blocks)
-                t, tr = timed(ctx, sc, cam, thr, n=3)
-                print("   steps %2d tris %d blocks/SM %2d: %.2f ms (trace %.2f)" % (steps, tris, blocks, t, tr), flush=True)
-            for k in ("LT_THREADED_NODE_STEPS", "LT_THREADED_TRI_TESTS", "LT_THREADED_BLOCKS_PER_SM"):
-                os.environ.pop(k, None)
         sc.release()
 
 
