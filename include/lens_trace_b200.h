@@ -222,6 +222,15 @@ int lt_debug_tile_rows(int height, int devices, int device, int32_t* out_rows, i
  * Exposed so that the layout can be checked against the reference traversal on a machine without a GPU. */
 int lt_debug_build_threaded(const void* nodes, uint64_t node_bytes, void* out_records);
 
+/* Host-only: the eight pruned copies lt_scene_upload builds beside those (same record format, inner nodes that
+ * cannot change which leaves a ray reaches left out; skip links index out_records).  *out_stride receives the
+ * records per copy; out_records (8 * stride * 32 bytes, at most 8 * node_count * 32) may be NULL to ask for it. */
+int lt_debug_build_threaded_pruned(const void* nodes, uint64_t node_bytes, void* out_records, int32_t* out_stride);
+
+/* Test hook: full != 0 makes launches on `scene` (single-GPU) walk the full threaded copies for every ray, 0 restores
+ * the pruned ones.  The output is the same either way; tests compare the two. */
+int lt_debug_scene_full_threaded(lt_scene* scene, int full);
+
 /* --- plug-in kernels: a user-written .cu file with the reference's kernel ABI (extern "C" __global__
  * linearKernel / tileKernel(LinearBVHNode*, Primitive*, Material*, LightContainer*, Camera*, float* out,
  * int width, int height, int depth), resources/kernels/cuda/basic.cu:331-340).  Replaces the NVRTC compile

@@ -86,7 +86,11 @@ static_assert(sizeof(LtTri) == 48, "triangle record is 48 bytes");
 // that sequence: the next record is the first node to visit after a box hit, `skip` the first node after
 // the subtree -- a traversal is `i = hit && inner ? i + 1 : skip` with no stack.  The bounds are stored
 // already selected by the octant's dirIsNeg (basic.cu:88-91), so the slab test needs no selects either.
-// One 32-byte sector, two 128-bit loads.
+// Host-built copies are followed by eight PRUNED copies (copy o at records prunedBase + o * prunedStride): the
+// same sequences without the inner nodes whose two child boxes lie inside their own box and which a ray that
+// entered the nearest kept ancestor usually enters too.  For a ray with finite, nonzero direction reciprocals and a
+// finite origin a contained child is hit only if its parent is, so the walk records the same leaves in the same
+// order; every other ray starts in the full copies.  One 32-byte sector, two 128-bit loads.
 struct __align__(16) LtThreadNode {
   float4 a;  // lo.x lo.y lo.z hi.x      lo = dirIsNeg ? boundsMax : boundsMin, hi the other one
   float4 b;  // hi.y hi.z bits(link) bits(skip)   link < 0: leaf, ~primitivesOffset; >= 0: inner node
@@ -108,7 +112,9 @@ struct LtSceneDev {
   int rootCount;              // primitiveCount of a leaf root (stats only)
   int stackDepth;             // entries a traversal stack needs (tree depth), <= 64
   int nodeCount, primCount, matCount;
-  const LtThreadNode* tnodes;  // 8 * nodeCount threaded records, or NULL (scene too large for the copies)
+  int prunedBase, prunedStride;  // pruned copy o of tnodes: records [prunedBase + o * prunedStride, + prunedStride);
+                                 // 0 and nodeCount: the full copies (tnodesCoherent, or no pruned copies)
+  const LtThreadNode* tnodes;  // 8 * nodeCount full threaded records, then the pruned ones, or NULL (scene too large)
   const LtThreadNode* tnodesCoherent;  // the same records for a large scene (built on the device), used only by the
                                        // lighting kernels' megakernel launches (camera rays + shadow rays towards a
                                        // light): incoherent rays spread over eight copies that no longer fit in L2

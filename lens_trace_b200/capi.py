@@ -17,7 +17,7 @@ LIB_PATH = os.path.join(_HERE, "liblt_b200.so")
 SYMBOLS = [
     "lt_api_version", "lt_ctx_create", "lt_ctx_destroy", "lt_last_error", "lt_ctx_set_stream", "lt_scene_upload",
     "lt_scene_release", "lt_render", "lt_render_device", "lt_accum_reset", "lt_accum_read", "lt_primary_hits",
-    "lt_last_stats", "lt_kernel_from_path", "lt_kernel_name", "lt_debug_random", "lt_debug_hemisphere", "lt_debug_build_threaded", "lt_plugin_load", "lt_render_plugin", "lt_primary_hits_flags", "lt_scene_build_lbvh", "lt_scene_download", "lt_scene_info",
+    "lt_last_stats", "lt_kernel_from_path", "lt_kernel_name", "lt_debug_random", "lt_debug_hemisphere", "lt_debug_build_threaded", "lt_debug_build_threaded_pruned", "lt_debug_scene_full_threaded", "lt_plugin_load", "lt_render_plugin", "lt_primary_hits_flags", "lt_scene_build_lbvh", "lt_scene_download", "lt_scene_info",
     "lt_debug_gather_peak", "lt_ctx_create_multi", "lt_ctx_device_count", "lt_host_register", "lt_host_unregister", "lt_debug_tile_rows",
 ]
 
@@ -86,6 +86,8 @@ def load():
     lib.lt_debug_random.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
     lib.lt_debug_hemisphere.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
     lib.lt_debug_build_threaded.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p]
+    lib.lt_debug_build_threaded_pruned.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.POINTER(C.c_int32)]
+    lib.lt_debug_scene_full_threaded.argtypes = [C.c_void_p, C.c_int]
     lib.lt_plugin_load.argtypes = [C.c_void_p, C.c_char_p, C.POINTER(C.c_int)]
     lib.lt_render_plugin.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                      C.c_int, C.c_int, C.c_void_p]
@@ -249,6 +251,11 @@ class Context:
                                                   iters, C.byref(gbs), C.byref(ns)), "lt_debug_gather_peak")
         return gbs.value, ns.value
 
+    def debug_full_threaded(self, scene, full):
+        """Test hook: every ray of later launches on `scene` walks the full threaded copies (full=True), or rays
+        with finite, nonzero reciprocals walk the pruned ones again (full=False, the default after upload)."""
+        self._check(self.lib.lt_debug_scene_full_threaded(scene.h, 1 if full else 0), "lt_debug_scene_full_threaded")
+
     def stats(self):
         s = Stats()
         self.lib.lt_last_stats(self.h, C.byref(s))
@@ -288,3 +295,16 @@ def build_threaded(nodes):
     if rc != 0:
         raise LtError("lt_debug_build_threaded failed (%d): %s" % (rc, lib.lt_last_error(None).decode()))
     return out
+
+
+def build_threaded_pruned(nodes):
+    """Host-only: the 8 x stride pruned threaded records lt_scene_upload builds beside the full ones
+    (lt_debug_build_threaded_pruned); skip links index the returned array flattened."""
+    lib = load()
+    nodes = np.ascontiguousarray(nodes)
+    stride = C.c_int32(0)
+    out = np.zeros((8, len(nodes)), THREAD_NODE)
+    rc = lib.lt_debug_build_threaded_pruned(nodes.ctypes.data, nodes.nbytes, out.ctypes.data, C.byref(stride))
+    if rc != 0:
+        raise LtError("lt_debug_build_threaded_pruned failed (%d): %s" % (rc, lib.lt_last_error(None).decode()))
+    return np.ascontiguousarray(out.reshape(-1)[:8 * stride.value].reshape(8, stride.value))

@@ -394,7 +394,8 @@ __device__ __forceinline__ bool trav_iter_lean(Trav& t, const LtSceneDev& sc, un
 }
 
 // ---- stackless traversal of the threaded tree (LtThreadNode, small scenes) -----------------------
-// Same box tests and triangle tests in the same order as the stack traversal above, hence the same hits:
+// Same triangle tests in the same order as the stack traversal above, hence the same hits, and the same box tests
+// (full copies) or a subset of them that cannot change which leaves are reached (pruned copies, see LtThreadNode):
 // the records of the ray's sign octant are laid out in visit order, so a step is one box test and
 // `cur = hit && inner ? cur + 1 : skip`.  No stack, no near/far selection, no per-axis min/max: the
 // record's bounds are already the dirIsNeg-selected ones, so for rays with finite reciprocals
@@ -405,8 +406,12 @@ __device__ __forceinline__ void trav_begin_threaded(Trav& t, const LtSceneDev& s
   t.iy = FRCP(t.r.dy);
   t.iz = FRCP(t.r.dz);
   t.negMask = (t.ix < 0.0f ? 1u : 0u) | (t.iy < 0.0f ? 2u : 0u) | (t.iz < 0.0f ? 4u : 0u);
-  const int rootRecord = (int)(t.negMask & 7u) * sc.nodeCount;  // the root record of the ray's octant copy
+  const int oct = (int)(t.negMask & 7u);
   if (!(finite3(t.ix, t.iy, t.iz) && finite3(t.r.ox, t.r.oy, t.r.oz))) t.negMask |= LT_EXACT_SLAB;
+  // the pruned copies rely on (b - o) * inv being monotonic in the bound b: not so for a non-finite reciprocal or
+  // origin, nor for a zero reciprocal (inf * 0 = NaN when b - o overflows); those rays walk the full copies
+  const bool full = (t.negMask & LT_EXACT_SLAB) || t.ix == 0.0f || t.iy == 0.0f || t.iz == 0.0f;
+  const int rootRecord = full ? oct * sc.nodeCount : sc.prunedBase + oct * sc.prunedStride;
   // every ray starts at the root: its box comes from the kernel parameters (constant bank) instead of a gather,
   // and an inner root that is hit continues at its near child, the next record of the copy
   t.cur = rootRecord;

@@ -97,7 +97,8 @@ struct lt_scene {
   RefLights* dLights = nullptr;
   LtWideNode* dWide = nullptr;
   LtTri* dTris = nullptr;
-  LtThreadNode* dThread = nullptr;  // 8 octant copies in visit order, small scenes only
+  LtThreadNode* dThread = nullptr;  // 8 octant copies in visit order, then 8 pruned ones, small scenes only
+  int threadStride = 0;             // records per pruned copy
   LtThreadNode* dThreadBig = nullptr;  // the same for a large scene, built on the device, for coherent-ray launches
   LtSceneDev dev = {};
 };
