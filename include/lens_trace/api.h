@@ -58,7 +58,10 @@ enum AccelerationStructureExplicitType {
   // --- B200 extension (not in the reference): LBVH built on the GPU (lt_scene_build_lbvh), same flattened layout
   ACCELERATION_STRUCTURE_TYPE_LBVH_B200 = 100,
   // --- B200 extension: host builder with binned surface-area-heuristic splits, same flattened layout
-  ACCELERATION_STRUCTURE_TYPE_SAH_B200 = 101
+  ACCELERATION_STRUCTURE_TYPE_SAH_B200 = 101,
+  // --- B200 extension: PLOC tree built on the GPU (lt_scene_build_ploc), same flattened layout; without a usable
+  // device the host SAH builder is used instead
+  ACCELERATION_STRUCTURE_TYPE_PLOC_B200 = 102
 };
 
 struct ThreadOrganizationOpenCL {

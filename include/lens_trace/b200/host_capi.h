@@ -16,7 +16,8 @@ void* lth_model_material_buffer(void* model);
 uint64_t lth_model_material_bytes(void* model);
 
 void* lth_as_create(void* model);
-/* type: 0 = host median-split (reference semantics), 100 = GPU LBVH (ACCELERATION_STRUCTURE_TYPE_LBVH_B200) */
+/* type: 0 = host median-split (reference semantics), 100 = GPU LBVH (ACCELERATION_STRUCTURE_TYPE_LBVH_B200),
+ * 101 = host binned SAH (ACCELERATION_STRUCTURE_TYPE_SAH_B200), 102 = GPU PLOC (ACCELERATION_STRUCTURE_TYPE_PLOC_B200) */
 void* lth_as_create_typed(void* model, int type);
 void lth_as_destroy(void* as);
 void* lth_as_node_buffer(void* as);

@@ -158,6 +158,11 @@ void lt_scene_release(lt_ctx* ctx, lt_scene* scene);
  * pointers, sizes in bytes: 32*(2n-1), 76*n, 260) so the CPU side can hold them. --- */
 int lt_scene_build_lbvh(lt_ctx* ctx, const void* primitives, uint64_t primitive_bytes, const void* materials,
                         uint64_t material_bytes, lt_scene** out_scene);
+/* The same contract with a PLOC tree (bottom-up clustering of mutual nearest neighbours over the Morton order,
+ * Meister & Bittner 2018): about the surface-area cost of the host SAH builder's tree at about the LBVH's build
+ * time (DESIGN.md section 4).  Deterministic.  Non-finite vertex coordinates -> LT_ERR_INVALID. */
+int lt_scene_build_ploc(lt_ctx* ctx, const void* primitives, uint64_t primitive_bytes, const void* materials,
+                        uint64_t material_bytes, lt_scene** out_scene);
 int lt_scene_download(lt_ctx* ctx, lt_scene* scene, void* nodes, uint64_t node_bytes, void* primitives,
                       uint64_t primitive_bytes, void* light_container);
 /* node and primitive counts of a scene */

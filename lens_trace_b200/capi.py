@@ -17,7 +17,7 @@ LIB_PATH = os.path.join(_HERE, "liblt_b200.so")
 SYMBOLS = [
     "lt_api_version", "lt_ctx_create", "lt_ctx_destroy", "lt_last_error", "lt_ctx_set_stream", "lt_scene_upload",
     "lt_scene_release", "lt_render", "lt_render_device", "lt_accum_reset", "lt_accum_read", "lt_primary_hits",
-    "lt_last_stats", "lt_kernel_from_path", "lt_kernel_name", "lt_debug_random", "lt_debug_hemisphere", "lt_debug_build_threaded", "lt_debug_build_threaded_pruned", "lt_debug_scene_full_threaded", "lt_plugin_load", "lt_render_plugin", "lt_primary_hits_flags", "lt_scene_build_lbvh", "lt_scene_download", "lt_scene_info",
+    "lt_last_stats", "lt_kernel_from_path", "lt_kernel_name", "lt_debug_random", "lt_debug_hemisphere", "lt_debug_build_threaded", "lt_debug_build_threaded_pruned", "lt_debug_scene_full_threaded", "lt_plugin_load", "lt_render_plugin", "lt_primary_hits_flags", "lt_scene_build_lbvh", "lt_scene_build_ploc", "lt_scene_download", "lt_scene_info",
     "lt_debug_gather_peak", "lt_ctx_create_multi", "lt_ctx_device_count", "lt_host_register", "lt_host_unregister", "lt_debug_tile_rows",
 ]
 
@@ -70,6 +70,7 @@ def load():
     lib.lt_scene_upload.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64,
                                     C.c_void_p, C.c_uint64, C.POINTER(C.c_void_p)]
     lib.lt_scene_build_lbvh.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.POINTER(C.c_void_p)]
+    lib.lt_scene_build_ploc.argtypes = lib.lt_scene_build_lbvh.argtypes
     lib.lt_scene_download.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p]
     lib.lt_scene_info.argtypes = [C.c_void_p, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_int32)]
     lib.lt_scene_release.argtypes = [C.c_void_p, C.c_void_p]
@@ -163,12 +164,19 @@ class Context:
 
     def build_lbvh(self, prims, materials):
         """Device-side LBVH over `prims` (layouts.PRIM array in any order) -> Scene handle"""
+        return self._build("lt_scene_build_lbvh", prims, materials)
+
+    def build_ploc(self, prims, materials):
+        """Device-side PLOC tree over `prims` (layouts.PRIM array in any order) -> Scene handle"""
+        return self._build("lt_scene_build_ploc", prims, materials)
+
+    def _build(self, entry, prims, materials):
         prims = np.ascontiguousarray(prims, dtype=L.PRIM)
         materials = np.ascontiguousarray(materials, dtype=L.MATERIAL)
         out = C.c_void_p()
-        rc = self.lib.lt_scene_build_lbvh(self.h, prims.ctypes.data, prims.nbytes, materials.ctypes.data,
-                                          materials.nbytes, C.byref(out))
-        self._check(rc, "lt_scene_build_lbvh")
+        rc = getattr(self.lib, entry)(self.h, prims.ctypes.data, prims.nbytes, materials.ctypes.data, materials.nbytes,
+                                      C.byref(out))
+        self._check(rc, entry)
         sc = Scene(self, out)
         sc.materials = materials.copy()
         return sc

@@ -10,6 +10,7 @@
 #include <string.h>
 
 #include <atomic>
+#include <cmath>
 #include <condition_variable>
 #include <mutex>
 #include <string>
@@ -495,28 +496,38 @@ static int finish_scene(lt_ctx* ctx, lt_scene* s, int nNodes, int nPrims, int nM
   return LT_OK;
 }
 
-extern "C" int lt_scene_build_lbvh(lt_ctx* ctx, const void* primitives, uint64_t primitive_bytes, const void* materials,
-                                   uint64_t material_bytes, lt_scene** out_scene) {
-  if (!ctx) return fail(nullptr, LT_ERR_INVALID, "lt_scene_build_lbvh: ctx is NULL");
-  if (ctx->group) return fail(ctx, LT_ERR_UNSUPPORTED, "lt_scene_build_lbvh: build on a single-GPU context, download, and upload to the multi-GPU context");
-  if (!out_scene || !primitives || !materials) return fail(ctx, LT_ERR_INVALID, "lt_scene_build_lbvh: NULL argument");
+// The device builders (lt_bvh.cu) behind lt_scene_build_lbvh and lt_scene_build_ploc: argument checks, upload of the
+// inputs, build, depth check and re-flatten.  `who` names the entry point in error messages.
+static int build_scene_on_device(lt_ctx* ctx, LtBvhBuilder builder, const char* who, const void* primitives,
+                                 uint64_t primitive_bytes, const void* materials, uint64_t material_bytes,
+                                 lt_scene** out_scene) {
+  const std::string w = std::string(who) + ": ";
+  if (!ctx) return fail(nullptr, LT_ERR_INVALID, w + "ctx is NULL");
+  if (ctx->group) return fail(ctx, LT_ERR_UNSUPPORTED, w + "build on a single-GPU context, download, and upload to the multi-GPU context");
+  if (!out_scene || !primitives || !materials) return fail(ctx, LT_ERR_INVALID, w + "NULL argument");
   *out_scene = nullptr;
   if (primitive_bytes == 0 || primitive_bytes % sizeof(RefPrim) || material_bytes == 0 ||
       material_bytes % sizeof(RefMaterial))
-    return fail(ctx, LT_ERR_INVALID, "lt_scene_build_lbvh: buffer size is not a multiple of the reference record size");
+    return fail(ctx, LT_ERR_INVALID, w + "buffer size is not a multiple of the reference record size");
   uint64_t nPrims = primitive_bytes / sizeof(RefPrim), nMats = material_bytes / sizeof(RefMaterial);
-  if (nPrims < 2) return fail(ctx, LT_ERR_UNSUPPORTED, "lt_scene_build_lbvh: needs at least two primitives");
-  if (nPrims > 0x3fffffffull) return fail(ctx, LT_ERR_INVALID, "lt_scene_build_lbvh: too many primitives");
+  if (nPrims < 2) return fail(ctx, LT_ERR_UNSUPPORTED, w + "needs at least two primitives");
+  if (nPrims > 0x3fffffffull) return fail(ctx, LT_ERR_INVALID, w + "too many primitives");
   const RefPrim* hPrims = (const RefPrim*)primitives;
   for (uint64_t i = 0; i < nPrims; i++)
     if (hPrims[i].materialIndex < 0 || (uint64_t)hPrims[i].materialIndex >= nMats)
-      return fail(ctx, LT_ERR_INVALID, "lt_scene_build_lbvh: primitive materialIndex out of range");
+      return fail(ctx, LT_ERR_INVALID, w + "primitive materialIndex out of range");
+  // PLOC compares box areas; its progress argument needs every area to be a number
+  if (builder == LT_BVH_PLOC)
+    for (uint64_t i = 0; i < nPrims; i++)
+      for (int k = 0; k < 3; k++)
+        if (!std::isfinite(hPrims[i].a[k]) || !std::isfinite(hPrims[i].b[k]) || !std::isfinite(hPrims[i].c[k]))
+          return fail(ctx, LT_ERR_INVALID, w + "non-finite vertex coordinate");
   CK(cudaSetDevice(ctx->device));
   int n = (int)nPrims, nNodes = 2 * n - 1;
   lt_scene* s = new lt_scene();
   RefPrim* dInput = nullptr;
   void* scratch = nullptr;
-  size_t scratchBytes = lt_bvh_scratch_bytes(n);
+  size_t scratchBytes = lt_bvh_scratch_bytes(n, builder);
   cudaError_t e = cudaSuccess;
   auto A = [&](cudaError_t r) { if (e == cudaSuccess) e = r; };
   A(cudaMalloc(&s->dNodes, sizeof(RefNode) * (size_t)nNodes));
@@ -531,8 +542,8 @@ extern "C" int lt_scene_build_lbvh(lt_ctx* ctx, const void* primitives, uint64_t
   A(cudaMemcpyAsync(s->dMats, materials, material_bytes, cudaMemcpyHostToDevice, st));
   int maxDepth = 0, launches = -1;
   if (e == cudaSuccess)
-    launches = lt_launch_bvh_build(dInput, n, s->dMats, (int)nMats, s->dNodes, s->dPrims, s->dLights, scratch, scratchBytes,
-                                   &maxDepth, st);
+    launches = lt_launch_bvh_build(builder, dInput, n, s->dMats, (int)nMats, s->dNodes, s->dPrims, s->dLights, scratch,
+                                   scratchBytes, &maxDepth, st);
   RefNode root;
   memset(&root, 0, sizeof root);
   if (e == cudaSuccess && launches >= 0) A(cudaMemcpy(&root, s->dNodes, sizeof root, cudaMemcpyDeviceToHost));
@@ -540,16 +551,28 @@ extern "C" int lt_scene_build_lbvh(lt_ctx* ctx, const void* primitives, uint64_t
   cudaFree(scratch);
   if (e != cudaSuccess || launches < 0) {
     lt_scene_release(ctx, s);
-    return fail(ctx, LT_ERR_CUDA, std::string("lt_scene_build_lbvh: ") + (e != cudaSuccess ? cudaGetErrorString(e) : "build failed"));
+    return fail(ctx, LT_ERR_CUDA, w + (e != cudaSuccess ? cudaGetErrorString(e) : "build failed"));
   }
   if (maxDepth > 64) {
     lt_scene_release(ctx, s);
-    return fail(ctx, LT_ERR_UNSUPPORTED, "lt_scene_build_lbvh: tree deeper than 64 (too many coincident centroids); use the host builder");
+    return fail(ctx, LT_ERR_UNSUPPORTED, w + "tree deeper than 64 (too many coincident centroids); use the host builder");
   }
-  int rc = finish_scene(ctx, s, nNodes, n, (int)nMats, root, maxDepth, "lt_scene_build_lbvh");
+  int rc = finish_scene(ctx, s, nNodes, n, (int)nMats, root, maxDepth, who);
   if (rc != LT_OK) return rc;
   *out_scene = s;
   return LT_OK;
+}
+
+extern "C" int lt_scene_build_lbvh(lt_ctx* ctx, const void* primitives, uint64_t primitive_bytes, const void* materials,
+                                   uint64_t material_bytes, lt_scene** out_scene) {
+  return build_scene_on_device(ctx, LT_BVH_LBVH, "lt_scene_build_lbvh", primitives, primitive_bytes, materials,
+                               material_bytes, out_scene);
+}
+
+extern "C" int lt_scene_build_ploc(lt_ctx* ctx, const void* primitives, uint64_t primitive_bytes, const void* materials,
+                                   uint64_t material_bytes, lt_scene** out_scene) {
+  return build_scene_on_device(ctx, LT_BVH_PLOC, "lt_scene_build_ploc", primitives, primitive_bytes, materials,
+                               material_bytes, out_scene);
 }
 
 extern "C" int lt_scene_download(lt_ctx* ctx, lt_scene* scene, void* nodes, uint64_t node_bytes, void* primitives,

@@ -120,8 +120,9 @@ int lt_internal_download(lt_ctx* ctx, float* host_out, const float* dSrc, size_t
 int lt_internal_render_rows(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params,
                             float* device_out, int fullHeight, int rowBlock, int rowStride, int rowPhase, int sync);
 
-// device-side LBVH construction in the reference's flattened layout (lt_bvh.cu)
-size_t lt_bvh_scratch_bytes(int n);
-int lt_launch_bvh_build(const RefPrim* dPrims, int n, const RefMaterial* dMats, int matCount, RefNode* dNodes,
-                        RefPrim* dOrderedPrims, RefLights* dLights, void* scratch, size_t scratchBytes, int* outMaxDepth,
-                        cudaStream_t stream);
+// device-side BVH construction in the reference's flattened layout (lt_bvh.cu)
+enum LtBvhBuilder { LT_BVH_LBVH, LT_BVH_PLOC };
+size_t lt_bvh_scratch_bytes(int n, LtBvhBuilder builder);
+int lt_launch_bvh_build(LtBvhBuilder builder, const RefPrim* dPrims, int n, const RefMaterial* dMats, int matCount,
+                        RefNode* dNodes, RefPrim* dOrderedPrims, RefLights* dLights, void* scratch, size_t scratchBytes,
+                        int* outMaxDepth, cudaStream_t stream);

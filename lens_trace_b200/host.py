@@ -106,6 +106,7 @@ class AccelerationStructure:
     HOST_MEDIAN_SPLIT = 0
     GPU_LBVH = 100
     HOST_SAH = 101
+    GPU_PLOC = 102
 
     def __init__(self, model, kind=0):
         self.lib = load()
@@ -190,7 +191,8 @@ def write_synthetic_scene(path, grid_n, seed=0x5EED):
 
 
 def load_scene_buffers(obj_path, kind=0):
-    """OBJ -> Model -> AccelerationStructureExplicit (kind: 0 median split, 100 GPU LBVH, 101 host SAH) -> flat
+    """OBJ -> Model -> AccelerationStructureExplicit (kind: 0 median split, 100 GPU LBVH, 101 host SAH,
+    102 GPU PLOC) -> flat
     buffers (layouts.SceneBuffers)."""
     m = Model(obj_path)
     if m.primitive_count == 0:

@@ -197,10 +197,12 @@ AccelerationStructureExplicit::AccelerationStructureExplicit(
   memset(&lightContainer, 0, sizeof lightContainer);
   if (infos.empty()) return;
 
-  // opt-in: build on the GPU (Morton-order LBVH, lens_trace_b200/csrc/lt_bvh.cu) and keep the result in the
-  // same host-side buffers; if no device is usable the host median-split build below is used instead
-  if (accelerationStructureExplicitProperties.accelerationStructureExplicitType == ACCELERATION_STRUCTURE_TYPE_LBVH_B200 &&
-      infos.size() >= 2) {
+  // opt-in: build on the GPU (Morton-order LBVH or PLOC, lens_trace_b200/csrc/lt_bvh.cu) and keep the result in the
+  // same host-side buffers; if no device is usable a host build below is used instead: the median split for the
+  // LBVH, the binned SAH (the closest tree in kind) for PLOC
+  const int type = accelerationStructureExplicitProperties.accelerationStructureExplicitType;
+  const bool ploc = type == ACCELERATION_STRUCTURE_TYPE_PLOC_B200;
+  if ((type == ACCELERATION_STRUCTURE_TYPE_LBVH_B200 || ploc) && infos.size() >= 2) {
     std::vector<Primitive> input(infos.size());
     for (size_t x = 0; x < infos.size(); x++) {
       memcpy(input[x].positionA, infos[x].positionA, sizeof(float) * 18);  // positions + normals are contiguous
@@ -208,9 +210,10 @@ AccelerationStructureExplicit::AccelerationStructureExplicit(
     }
     lt_ctx* ctx = nullptr;
     lt_scene* scene = nullptr;
+    auto build = ploc ? lt_scene_build_ploc : lt_scene_build_lbvh;
     bool ok = lt_ctx_create(0, &ctx) == LT_OK &&
-              lt_scene_build_lbvh(ctx, input.data(), input.size() * sizeof(Primitive), materials,
-                                  materialCount * sizeof(Material), &scene) == LT_OK;
+              build(ctx, input.data(), input.size() * sizeof(Primitive), materials, materialCount * sizeof(Material),
+                    &scene) == LT_OK;
     if (ok) {
       linearNodes.resize(2 * infos.size() - 1);
       orderedPrimitives.resize(infos.size());
@@ -218,7 +221,8 @@ AccelerationStructureExplicit::AccelerationStructureExplicit(
                              orderedPrimitives.data(), orderedPrimitives.size() * sizeof(Primitive),
                              &lightContainer) == LT_OK;
     }
-    if (!ok) printf("WARNING: GPU BVH build unavailable (%s); using the host builder\n", lt_last_error(ctx));
+    if (!ok)
+      printf("WARNING: GPU BVH build unavailable (%s); using the host %sbuilder\n", lt_last_error(ctx), ploc ? "SAH " : "");
     if (scene) lt_scene_release(ctx, scene);
     if (ctx) lt_ctx_destroy(ctx);
     if (ok) return;
@@ -230,7 +234,7 @@ AccelerationStructureExplicit::AccelerationStructureExplicit(
   Builder b(infos, linearNodes);
   // opt-in: binned-SAH splits instead of the reference's median split (same layout, same kernels, fewer box tests
   // per ray; a different tree, so never the parity configuration)
-  b.sah = accelerationStructureExplicitProperties.accelerationStructureExplicitType == ACCELERATION_STRUCTURE_TYPE_SAH_B200;
+  b.sah = type == ACCELERATION_STRUCTURE_TYPE_SAH_B200 || ploc;
   b.build(0, (int)infos.size());
 
   orderedPrimitives.resize(infos.size());
