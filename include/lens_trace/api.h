@@ -456,9 +456,12 @@ public:
   void forgetScenes();  // drops every cached device scene
   size_t cachedSceneCount() const { return sceneCache.size(); }
 
+  // workBlockSize: the OpenCL work block of a user-written .cl kernel (NULL or 0: the whole image); blockSize is then
+  // its work-group size (0: the library's choice).  The built-in pipelines ignore the work block.
   void renderCommon(const std::string& kernelFilePath, KernelMode kernelMode, const uint64_t blockSize[2],
                     const uint64_t imageDimensions[3], void* pOutputBuffer, uint64_t outputBufferSize,
-                    void* pAccelerationStructureExplicit, void* pModel, void* pCamera, void* pNext);
+                    void* pAccelerationStructureExplicit, void* pModel, void* pCamera, void* pNext,
+                    const uint64_t* workBlockSize = nullptr);
 };
 
 // ================================================================================================

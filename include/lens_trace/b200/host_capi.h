@@ -45,6 +45,13 @@ uint64_t lth_renderer_cached_scenes(void* renderer, int platform);
 void lth_render(void* renderer, int platform, const char* kernel_file_path, int kernel_mode, int thread_org_mode,
                 uint64_t bx, uint64_t by, uint64_t width, uint64_t height, uint64_t depth, float* out,
                 uint64_t out_bytes, void* as, void* model, void* camera, void* ext);
+/* RendererOpenCL::render with the work block and the work-group size given apart (lth_render gives both the same
+ * value): thread_org_mode 0 = MAX_FIT, 1 = CUSTOM with workBlockSize (work_bx, work_by) and threadGroupSize
+ * (group_x, group_y).  The work block matters to user-written .cl kernels only. */
+void lth_render_opencl(void* renderer, const char* kernel_file_path, int kernel_mode, int thread_org_mode,
+                       uint64_t work_bx, uint64_t work_by, uint64_t group_x, uint64_t group_y, uint64_t width,
+                       uint64_t height, uint64_t depth, float* out, uint64_t out_bytes, void* as, void* model,
+                       void* camera, void* ext);
 
 uint64_t lth_write_synthetic_scene(const char* obj_path, uint32_t grid_n, uint64_t seed);
 

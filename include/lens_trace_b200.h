@@ -246,11 +246,38 @@ int lt_plugin_load(lt_ctx* ctx, const char* kernel_file_path, int* out_plugin_id
 int lt_render_plugin(lt_ctx* ctx, lt_scene* scene, const void* camera28, int plugin_id, int kernel_mode, int width,
                      int height, int depth, int block_x, int block_y, float* host_out);
 
+/* --- OpenCL C plug-ins: lt_plugin_load on a path ending in ".cl" translates the file onto this library's OpenCL C
+ * runtime (the subset of INTEGRATION.md: vector types, math / geometric / work-item built-ins; no __local memory,
+ * barriers, images, atomics or half) and compiles it with NVRTC for sm_100a, once per context.  Every
+ * `__kernel void linearKernel` / `tileKernel` of the file must take the reference's OpenCL arguments
+ *   (LinearBVHNode*, Primitive*, Material*, LightContainer*, Camera*, float* output, uint currentBlock, uint W,
+ *    uint H, uint depth)
+ * under the user's own struct names, or the file does not compile.  `#pragma OPENCL FP_CONTRACT OFF` anywhere in the
+ * file compiles all of it without contraction (default: a * b + c may fuse, as OpenCL C allows).  A compile error
+ * returns LT_ERR_UNSUPPORTED with the NVRTC log, which names the user's file and line.
+ * lt_render_plugin_cl launches it like the reference's OpenCL backend (src/opencl/renderer_opencl.cpp:84-146): one
+ * launch per work block, (width / work_block_x) * (height / work_block_y) of them (integer division), global size =
+ * the work block, local size = group, currentBlock = the block's index.  A work block of 0 is the whole image in that
+ * dimension (what THREAD_ORGANIZATION_MODE_MAX_FIT renders); group 0 x 0 is the library's choice, any other group
+ * must divide the work block (LT_ERR_INVALID otherwise).  Pixels no block covers are written as 0.  Synchronous;
+ * lt_stats.kernel_ms and kernel_launches describe the call.  lt_render_plugin on a .cl plug-in and
+ * lt_render_plugin_cl on a .cu plug-in return LT_ERR_INVALID. --- */
+int lt_render_plugin_cl(lt_ctx* ctx, lt_scene* scene, const void* camera28, int plugin_id, int kernel_mode, int width,
+                        int height, int depth, int work_block_x, int work_block_y, int group_x, int group_y,
+                        float* host_out);
+/* Host-only (NVRTC, no device or driver needed): translate and compile a .cl file as lt_plugin_load would.  Returns 0,
+ * or LT_ERR_UNSUPPORTED with the reason / NVRTC log copied into log (NUL-terminated, truncated to log_bytes). */
+int lt_debug_compile_cl(const char* kernel_file_path, char* log, uint64_t log_bytes);
+/* Host-only: the translation of OpenCL C text that lt_debug_compile_cl compiles (before the runtime header and the
+ * generated entry points are added).  Returns the bytes needed including the NUL; out receives the text when out_bytes
+ * suffices.  *contract_off (may be NULL) = 1 when the text turns FP contraction off. */
+int64_t lt_debug_translate_cl(const char* text, char* out, uint64_t out_bytes, int32_t* contract_off);
+
 /* Maps RenderProperties*::kernelFilePath to an lt_kernel by the file's CONTENT: a descriptor file of this
  * repository (comment lines only, one reading "lt-pipeline: <tag>") or the unmodified text of one of the seven
  * kernel files the reference ships (content hash) selects the built-in pipeline that reproduces it.  Any other
  * file -- including an edited copy of a shipped kernel under its old name -- returns LT_ERR_UNSUPPORTED: the
- * renderer compiles such a .cu as a plug-in (lt_plugin_load) and reports an error for a .cl. */
+ * renderer compiles such a file as a plug-in (lt_plugin_load), a .cu as CUDA and a .cl as OpenCL C. */
 int lt_kernel_from_path(const char* kernel_file_path);
 const char* lt_kernel_name(int kernel);
 

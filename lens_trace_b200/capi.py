@@ -17,7 +17,7 @@ LIB_PATH = os.path.join(_HERE, "liblt_b200.so")
 SYMBOLS = [
     "lt_api_version", "lt_ctx_create", "lt_ctx_destroy", "lt_last_error", "lt_ctx_set_stream", "lt_scene_upload",
     "lt_scene_release", "lt_render", "lt_render_device", "lt_accum_reset", "lt_accum_read", "lt_primary_hits",
-    "lt_last_stats", "lt_kernel_from_path", "lt_kernel_name", "lt_debug_random", "lt_debug_hemisphere", "lt_debug_build_threaded", "lt_debug_build_threaded_pruned", "lt_debug_scene_full_threaded", "lt_plugin_load", "lt_render_plugin", "lt_primary_hits_flags", "lt_scene_build_lbvh", "lt_scene_build_ploc", "lt_scene_download", "lt_scene_info",
+    "lt_last_stats", "lt_kernel_from_path", "lt_kernel_name", "lt_debug_random", "lt_debug_hemisphere", "lt_debug_build_threaded", "lt_debug_build_threaded_pruned", "lt_debug_scene_full_threaded", "lt_plugin_load", "lt_render_plugin", "lt_render_plugin_cl", "lt_debug_compile_cl", "lt_debug_translate_cl", "lt_primary_hits_flags", "lt_scene_build_lbvh", "lt_scene_build_ploc", "lt_scene_download", "lt_scene_info",
     "lt_debug_gather_peak", "lt_ctx_create_multi", "lt_ctx_device_count", "lt_host_register", "lt_host_unregister", "lt_debug_tile_rows",
 ]
 
@@ -92,6 +92,10 @@ def load():
     lib.lt_plugin_load.argtypes = [C.c_void_p, C.c_char_p, C.POINTER(C.c_int)]
     lib.lt_render_plugin.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                      C.c_int, C.c_int, C.c_void_p]
+    lib.lt_render_plugin_cl.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p] + [C.c_int] * 9 + [C.c_void_p]
+    lib.lt_debug_compile_cl.argtypes = [C.c_char_p, C.c_char_p, C.c_uint64]
+    lib.lt_debug_translate_cl.argtypes = [C.c_char_p, C.c_char_p, C.c_uint64, C.POINTER(C.c_int32)]
+    lib.lt_debug_translate_cl.restype = C.c_int64
     lib.lt_debug_gather_peak.argtypes = [C.c_void_p, C.c_uint64, C.c_int, C.c_int, C.c_int, C.c_int,
                                          C.POINTER(C.c_double), C.POINTER(C.c_double)]
     lib.lt_kernel_from_path.argtypes = [C.c_char_p]
@@ -103,6 +107,24 @@ def load():
 
 def kernel_from_path(path):
     return load().lt_kernel_from_path(path.encode())
+
+
+def compile_cl(path, log_bytes=1 << 20):
+    """Translate and compile an OpenCL C kernel file for sm_100a as lt_plugin_load would, without a device.
+    Returns (ok, log): the log holds the reason or the NVRTC messages, which name the file and line."""
+    log = C.create_string_buffer(log_bytes)
+    rc = load().lt_debug_compile_cl(path.encode(), log, log_bytes)
+    return rc == 0, log.value.decode(errors="replace")
+
+
+def translate_cl(text):
+    """The library's translation of OpenCL C text (see lt_debug_translate_cl): (translated text, contraction off)."""
+    lib = load()
+    off = C.c_int32(0)
+    n = lib.lt_debug_translate_cl(text.encode(), None, 0, C.byref(off))
+    buf = C.create_string_buffer(n)
+    lib.lt_debug_translate_cl(text.encode(), buf, n, C.byref(off))
+    return buf.value.decode(), bool(off.value)
 
 
 def make_params(kernel, width, height, depth=3, kernel_mode=0, max_ray_depth=0, frames=1, frame_stride=1,
@@ -236,6 +258,17 @@ class Context:
         cam = np.ascontiguousarray(camera, dtype=L.CAMERA)
         self._check(self.lib.lt_render_plugin(self.h, scene.h, cam.ctypes.data, plugin_id, kernel_mode, width, height,
                                               depth, block[0], block[1], out.ctypes.data), "lt_render_plugin")
+        return out
+
+    def render_plugin_cl(self, scene, camera, plugin_id, width, height, depth=3, kernel_mode=0, work_block=(0, 0),
+                         group=(0, 0)):
+        """An OpenCL C plug-in (a .cl file given to plugin_load), launched as the reference's OpenCL backend does: one
+        launch per work block ((0, 0) = the whole image), work-group `group` ((0, 0) = the library's choice)."""
+        out = np.zeros((height, width, depth), dtype=np.float32)
+        cam = np.ascontiguousarray(camera, dtype=L.CAMERA)
+        self._check(self.lib.lt_render_plugin_cl(self.h, scene.h, cam.ctypes.data, plugin_id, kernel_mode, width, height,
+                                                 depth, work_block[0], work_block[1], group[0], group[1],
+                                                 out.ctypes.data), "lt_render_plugin_cl")
         return out
 
     def debug_random(self, fx, fy, seed):

@@ -971,6 +971,9 @@ extern "C" int lt_render_plugin(lt_ctx* ctx, lt_scene* scene, const void* camera
   if (!scene || !camera28 || plugin_id < 0 || plugin_id >= (int)ctx->plugins.size() || width <= 0 || height <= 0 ||
       depth < 1)
     return fail(ctx, LT_ERR_INVALID, "lt_render_plugin: bad argument");
+  if (lt_plugin_is_opencl_c(ctx->plugins[plugin_id]))
+    return fail(ctx, LT_ERR_INVALID, "lt_render_plugin: plug-in " + std::to_string(plugin_id) +
+                                         " is an OpenCL C kernel; launch it with lt_render_plugin_cl");
   CK(cudaSetDevice(ctx->device));
   size_t floats = (size_t)width * height * depth;
   int rc = ensure_out(ctx, floats);
@@ -988,6 +991,65 @@ extern "C" int lt_render_plugin(lt_ctx* ctx, lt_scene* scene, const void* camera
   CK(cudaEventElapsedTime(&ctx->stats.kernel_ms, ctx->ev0, ctx->ev1));
   ctx->stats.kernel_launches = 1;
   if (host_out) return download(ctx, host_out, ctx->dOut, floats * sizeof(float));
+  return LT_OK;
+}
+
+extern "C" int lt_render_plugin_cl(lt_ctx* ctx, lt_scene* scene, const void* camera28, int plugin_id, int kernel_mode,
+                                   int width, int height, int depth, int work_block_x, int work_block_y, int group_x,
+                                   int group_y, float* host_out) {
+  if (!ctx) return fail(nullptr, LT_ERR_INVALID, "lt_render_plugin_cl: ctx is NULL");
+  if (ctx->group) return fail(ctx, LT_ERR_UNSUPPORTED, "lt_render_plugin_cl: plug-in kernels run on single-GPU contexts");
+  if (!scene || !camera28 || plugin_id < 0 || plugin_id >= (int)ctx->plugins.size() || width <= 0 || height <= 0 ||
+      depth < 1)
+    return fail(ctx, LT_ERR_INVALID, "lt_render_plugin_cl: bad argument");
+  if (!lt_plugin_is_opencl_c(ctx->plugins[plugin_id]))
+    return fail(ctx, LT_ERR_INVALID, "lt_render_plugin_cl: plug-in " + std::to_string(plugin_id) +
+                                         " is a CUDA kernel; launch it with lt_render_plugin");
+  std::string err;
+  int wbx = work_block_x, wby = work_block_y, gx = group_x, gy = group_y;
+  if (!lt_plugin_cl_shape(width, height, &wbx, &wby, &gx, &gy, &err))
+    return fail(ctx, LT_ERR_INVALID, "lt_render_plugin_cl: " + err);
+  CK(cudaSetDevice(ctx->device));
+  size_t floats = (size_t)width * height * depth;
+  int rc = ensure_out(ctx, floats);
+  if (rc != LT_OK) return rc;
+  if (!ctx->dCamera) CK(cudaMalloc(&ctx->dCamera, sizeof(RefCamera)));
+  CK(cudaMemcpyAsync(ctx->dCamera, camera28, sizeof(RefCamera), cudaMemcpyHostToDevice, ctx->stream));
+  // pixels outside every work block (the remainder of W / wbx and H / wby) read 0; the reference leaves them undefined
+  CK(cudaMemsetAsync(ctx->dOut, 0, floats * sizeof(float), ctx->stream));
+  CK(cudaEventRecord(ctx->ev0, ctx->stream));
+  int launches = lt_plugin_launch_cl(ctx->plugins[plugin_id], kernel_mode ? 1 : 0, scene->dNodes, scene->dPrims,
+                                     scene->dMats, scene->dLights, ctx->dCamera, ctx->dOut, width, height, depth, wbx, wby,
+                                     gx, gy, ctx->stream, &err);
+  if (launches < 0) return fail(ctx, LT_ERR_CUDA, "lt_render_plugin_cl: " + err);
+  CK(cudaEventRecord(ctx->ev1, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  CK(cudaEventElapsedTime(&ctx->stats.kernel_ms, ctx->ev0, ctx->ev1));
+  ctx->stats.kernel_launches = launches;
+  if (host_out) return download(ctx, host_out, ctx->dOut, floats * sizeof(float));
+  return LT_OK;
+}
+
+extern "C" int64_t lt_debug_translate_cl(const char* text, char* out, uint64_t out_bytes, int32_t* contract_off) {
+  if (!text) return fail(nullptr, LT_ERR_INVALID, "lt_debug_translate_cl: NULL text");
+  bool off = false;
+  std::vector<std::pair<std::string, int>> kernels;
+  std::string t = lt_cl_translate(text, &off, &kernels);
+  if (contract_off) *contract_off = off ? 1 : 0;
+  if (out && out_bytes > t.size()) memcpy(out, t.c_str(), t.size() + 1);
+  return (int64_t)t.size() + 1;
+}
+
+extern "C" int lt_debug_compile_cl(const char* kernel_file_path, char* log, uint64_t log_bytes) {
+  if (!kernel_file_path) return fail(nullptr, LT_ERR_INVALID, "lt_debug_compile_cl: NULL path");
+  std::string err;
+  bool ok = lt_plugin_compile_cl_only(kernel_file_path, &err);
+  if (log && log_bytes) {
+    size_t n = err.size() < log_bytes - 1 ? err.size() : (size_t)(log_bytes - 1);
+    memcpy(log, err.data(), n);
+    log[n] = 0;
+  }
+  if (!ok) return fail(nullptr, LT_ERR_UNSUPPORTED, "lt_debug_compile_cl: " + err);
   return LT_OK;
 }
 
@@ -1127,8 +1189,8 @@ extern "C" const char* lt_kernel_name(int kernel) {
 //   * a file whose text is, byte for byte (CR dropped), one of the seven kernel files the reference ships
 //     (lt_kernel_hashes.inc: FNV-1a-64 + length; only hashes are stored)
 // maps to the hand-written pipeline that reproduces that kernel.  Anything else -- including an EDITED copy of a
-// shipped kernel under its old name -- is a user kernel: LT_ERR_UNSUPPORTED here; the renderer then compiles a .cu
-// as a plug-in (lt_plugin_load) and reports an error for a .cl (OpenCL C cannot be compiled for sm_100a here).
+// shipped kernel under its old name -- is a user kernel: LT_ERR_UNSUPPORTED here; the renderer then compiles it as a
+// plug-in (lt_plugin_load): a .cu as CUDA, a .cl as OpenCL C on the runtime of lt_opencl_c.cuh.
 struct LtKernelHash {
   unsigned long long hash;
   size_t bytes;
@@ -1194,6 +1256,6 @@ extern "C" int lt_kernel_from_path(const char* path) {
   for (size_t k = 0; k < sizeof kShippedKernels / sizeof kShippedKernels[0]; k++)
     if (kShippedKernels[k].hash == h && kShippedKernels[k].bytes == bytes) return kShippedKernels[k].kernel;
   g_error = std::string("lt_kernel_from_path: '") + path + "' is neither a kernel descriptor nor the unmodified text of "
-            "a shipped kernel (user kernels: .cu files are compiled as plug-ins, .cl files are not supported)";
+            "a shipped kernel (user kernels are compiled as plug-ins: lt_plugin_load)";
   return LT_ERR_UNSUPPORTED;
 }

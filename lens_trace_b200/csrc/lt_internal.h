@@ -50,12 +50,23 @@ int lt_launch_render_wavefront(const LtSceneDev& sc, const LtLaunch& L, float* d
 
 // user-written CUDA kernels with the reference's plug-in ABI (lt_plugin.cu)
 #include <string>
+#include <utility>
+#include <vector>
 struct LtPlugin;
 LtPlugin* lt_plugin_compile(const char* path, std::string* err);
 void lt_plugin_free(LtPlugin* p);
 int lt_plugin_launch(LtPlugin* p, int kernelMode, const LtSceneDev* sceneDev, const void* dNodes, const void* dPrims,
                      const void* dMats, const void* dLights, const void* dCamera, float* dOut, int width, int height,
                      int depth, int bx, int by, cudaStream_t stream, std::string* err);
+// user-written OpenCL C kernels (.cl): translated onto lt_opencl_c.cuh, compiled by NVRTC, launched like the reference's
+// OpenCL backend launches them
+bool lt_plugin_is_opencl_c(const LtPlugin* p);
+bool lt_plugin_compile_cl_only(const char* path, std::string* err);  // NVRTC only, no driver
+std::string lt_cl_translate(const std::string& src, bool* contractOff, std::vector<std::pair<std::string, int>>* kernels);
+bool lt_plugin_cl_shape(int width, int height, int* wbx, int* wby, int* gx, int* gy, std::string* err);
+int lt_plugin_launch_cl(LtPlugin* p, int kernelMode, const void* dNodes, const void* dPrims, const void* dMats,
+                        const void* dLights, const void* dCamera, float* dOut, int width, int height, int depth, int wbx,
+                        int wby, int gx, int gy, cudaStream_t stream, std::string* err);
 
 // ---- context and scene objects behind the C-ABI handles (lt_capi.cu; lt_multi.cu for multi-GPU contexts) ----
 #include <vector>

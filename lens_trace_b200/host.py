@@ -20,7 +20,7 @@ SYMBOLS = [
     "lth_as_primitive_buffer", "lth_as_primitive_bytes", "lth_as_light_buffer", "lth_as_light_bytes",
     "lth_camera_create", "lth_camera_destroy", "lth_camera_buffer", "lth_camera_set_frame_count",
     "lth_camera_increment_frame_count", "lth_camera_set_position", "lth_camera_set_rotation", "lth_renderer_create",
-    "lth_renderer_destroy", "lth_renderer_cached_scenes", "lth_render", "lth_write_synthetic_scene", "lth_run_scene_file",
+    "lth_renderer_destroy", "lth_renderer_cached_scenes", "lth_render", "lth_write_synthetic_scene", "lth_run_scene_file", "lth_render_opencl",
 ]
 
 
@@ -72,6 +72,9 @@ def load():
     lib.lth_render.argtypes = [vp, C.c_int, C.c_char_p, C.c_int, C.c_int, u64, u64, u64, u64, u64, vp, u64, vp, vp, vp,
                                vp]
     lib.lth_render.restype = None
+    lib.lth_render_opencl.argtypes = [vp, C.c_char_p, C.c_int, C.c_int, u64, u64, u64, u64, u64, u64, u64, vp, u64, vp,
+                                      vp, vp, vp]
+    lib.lth_render_opencl.restype = None
     lib.lth_write_synthetic_scene.argtypes = [C.c_char_p, C.c_uint32, u64]
     lib.lth_run_scene_file.argtypes = [C.c_char_p, vp, u64, C.POINTER(u64 * 3)]
     _lib = lib
@@ -156,10 +159,19 @@ class Renderer:
         self.h = self.lib.lth_renderer_create(platform)
 
     def render(self, kernel_file_path, width, height, accel, model, camera, depth=3, kernel_mode=0, block=None,
-               ext=None, out=None):
+               ext=None, out=None, work_block=None):
+        """block: CUDA block size, or OpenCL work-group size.  work_block (RendererOpenCL only): the OpenCL work block
+        of THREAD_ORGANIZATION_MODE_CUSTOM, with `block` as its work-group size (None: the library's choice)."""
         if out is None:
             out = np.zeros((height, width, depth), dtype=np.float32)
         bx, by = block if block else (0, 0)
+        if work_block is not None:
+            if self.platform != PLATFORM_OPENCL:
+                raise ValueError("work_block is a RendererOpenCL setting")
+            self.lib.lth_render_opencl(self.h, kernel_file_path.encode(), kernel_mode, 1, work_block[0], work_block[1],
+                                       bx, by, width, height, depth, out.ctypes.data, out.nbytes, accel.h, model.h,
+                                       camera.h, C.addressof(ext) if ext is not None else None)
+            return out
         self.lib.lth_render(self.h, self.platform, kernel_file_path.encode(), kernel_mode, 1 if block else 0, bx, by,
                             width, height, depth, out.ctypes.data, out.nbytes, accel.h, model.h, camera.h,
                             C.addressof(ext) if ext is not None else None)

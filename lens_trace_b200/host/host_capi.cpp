@@ -111,6 +111,32 @@ void lth_render(void* renderer, int platform, const char* kernel_file_path, int 
   }
 }
 
+void lth_render_opencl(void* renderer, const char* kernel_file_path, int kernel_mode, int thread_org_mode,
+                       uint64_t work_bx, uint64_t work_by, uint64_t group_x, uint64_t group_y, uint64_t width,
+                       uint64_t height, uint64_t depth, float* out, uint64_t out_bytes, void* as, void* model,
+                       void* camera, void* ext) {
+  RenderPropertiesOpenCL p = {};
+  p.sType = STRUCTURE_TYPE_RENDER_PROPERTIES_OPENCL;
+  p.pNext = ext;
+  p.kernelFilePath = kernel_file_path;
+  p.kernelMode = kernel_mode ? KERNEL_MODE_TILE : KERNEL_MODE_LINEAR;
+  p.threadOrganizationMode = thread_org_mode ? THREAD_ORGANIZATION_MODE_CUSTOM : THREAD_ORGANIZATION_MODE_MAX_FIT;
+  if (thread_org_mode) {
+    p.threadOrganization.sType = STRUCTURE_TYPE_THREAD_ORGANIZATION_OPENCL;
+    p.threadOrganization.workBlockSize[0] = work_bx;
+    p.threadOrganization.workBlockSize[1] = work_by;
+    p.threadOrganization.threadGroupSize[0] = group_x;
+    p.threadOrganization.threadGroupSize[1] = group_y;
+  }
+  p.imageDimensions[0] = width; p.imageDimensions[1] = height; p.imageDimensions[2] = depth;
+  p.pOutputBuffer = out;
+  p.outputBufferSize = out_bytes;
+  p.pAccelerationStructureExplicit = as;
+  p.pModel = model;
+  p.pCamera = camera;
+  ((RendererOpenCL*)renderer)->render(&p);
+}
+
 uint64_t lth_write_synthetic_scene(const char* obj_path, uint32_t grid_n, uint64_t seed) {
   return lt::writeSyntheticScene(obj_path, grid_n, seed);
 }

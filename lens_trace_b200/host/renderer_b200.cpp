@@ -73,7 +73,8 @@ void RendererB200::forgetScenes() {
 
 void RendererB200::renderCommon(const std::string& kernelFilePath, KernelMode kernelMode, const uint64_t blockSize[2],
                                 const uint64_t imageDimensions[3], void* pOutputBuffer, uint64_t outputBufferSize,
-                                void* pAccelerationStructureExplicit, void* pModel, void* pCamera, void* pNext) {
+                                void* pAccelerationStructureExplicit, void* pModel, void* pCamera, void* pNext,
+                                const uint64_t* workBlockSize) {
   if (!ctx) {
     printf("ERROR: no B200 context; nothing rendered (there is no CPU fallback)\n");
     return;
@@ -95,16 +96,19 @@ void RendererB200::renderCommon(const std::string& kernelFilePath, KernelMode ke
     kernel = lt_kernel_from_path(resolved == "INVALID RESOURCE" ? kernelFilePath.c_str() : resolved.c_str());
     kernelCache[kernelFilePath] = kernel;
   }
-  // not one of the shipped kernels: a user-written .cu with the reference's kernel ABI is compiled
-  // (once) with NVRTC for sm_100a and launched like the reference launches it; anything else is an error
+  // not one of the shipped kernels: a user-written .cu with the reference's CUDA kernel ABI, or a .cl with its
+  // OpenCL one, is compiled (once) with NVRTC for sm_100a and launched like the reference launches it; anything
+  // else is an error
   int plugin = -1;
+  bool isCl = false;
   if (kernel < 0) {
     std::string resolved = Resource::findResource(kernelFilePath);
     bool isCu = resolved.size() > 3 && resolved.compare(resolved.size() - 3, 3, ".cu") == 0;
+    isCl = resolved.size() > 3 && resolved.compare(resolved.size() - 3, 3, ".cl") == 0;
     std::map<std::string, int>::iterator pc = pluginCache.find(kernelFilePath);
     if (pc != pluginCache.end()) {
       plugin = pc->second;
-    } else if (isCu) {
+    } else if (isCu || isCl) {
       if (lt_plugin_load(ctx, resolved.c_str(), &plugin) != LT_OK) {
         printf("%s\n", lt_last_error(ctx));
         plugin = -1;
@@ -113,7 +117,7 @@ void RendererB200::renderCommon(const std::string& kernelFilePath, KernelMode ke
     }
     if (plugin < 0) {
       printf("Kernel Error: '%s' is not a kernel this renderer provides (%s)\n", kernelFilePath.c_str(),
-             isCu ? "plug-in compilation failed" : "only the shipped kernels and CUDA plug-ins are supported");
+             isCu || isCl ? "plug-in compilation failed" : "only the shipped kernels and .cu / .cl plug-ins are supported");
       return;
     }
   }
@@ -231,10 +235,17 @@ void RendererB200::renderCommon(const std::string& kernelFilePath, KernelMode ke
            (unsigned long long)need);
     return;
   }
-  int rc = plugin >= 0
-               ? lt_render_plugin(ctx, scene, camera->getCameraBuffer(), plugin, params.kernel_mode, params.width,
-                                  params.height, params.depth, params.block_x, params.block_y, (float*)pOutputBuffer)
-               : lt_render(useCtx, scene, camera->getCameraBuffer(), &params, (float*)pOutputBuffer);
+  int rc;
+  if (plugin >= 0 && isCl)
+    rc = lt_render_plugin_cl(ctx, scene, camera->getCameraBuffer(), plugin, params.kernel_mode, params.width,
+                             params.height, params.depth, workBlockSize ? (int)workBlockSize[0] : 0,
+                             workBlockSize ? (int)workBlockSize[1] : 0, params.block_x, params.block_y,
+                             (float*)pOutputBuffer);
+  else if (plugin >= 0)
+    rc = lt_render_plugin(ctx, scene, camera->getCameraBuffer(), plugin, params.kernel_mode, params.width,
+                          params.height, params.depth, params.block_x, params.block_y, (float*)pOutputBuffer);
+  else
+    rc = lt_render(useCtx, scene, camera->getCameraBuffer(), &params, (float*)pOutputBuffer);
   if (rc != LT_OK) {
     printf("Kernel Error: %d (%s)\n", rc, lt_last_error(useCtx));
     return;
@@ -272,15 +283,18 @@ RendererOpenCL::~RendererOpenCL() { delete impl; }
 void RendererOpenCL::render(void* pRenderProperties) {
   RenderPropertiesOpenCL* p = (RenderPropertiesOpenCL*)pRenderProperties;
   if (p->sType != STRUCTURE_TYPE_RENDER_PROPERTIES_OPENCL) printf("ERROR: RenderPropertiesOpenCL sType\n");
-  uint64_t block[2] = {0, 0};
+  uint64_t block[2] = {0, 0}, workBlock[2] = {0, 0};
   if (p->threadOrganizationMode == THREAD_ORGANIZATION_MODE_CUSTOM) {
     if (p->threadOrganization.sType != STRUCTURE_TYPE_THREAD_ORGANIZATION_OPENCL)
       printf("ERROR: ThreadOrganizationOpenCL sType\n");
     block[0] = p->threadOrganization.threadGroupSize[0];
     block[1] = p->threadOrganization.threadGroupSize[1];
+    workBlock[0] = p->threadOrganization.workBlockSize[0];
+    workBlock[1] = p->threadOrganization.workBlockSize[1];
   }
-  // The reference splits the image into work blocks and drops the remainder
-  // (src/opencl/renderer_opencl.cpp:90); the whole image is rendered here.
+  // The reference splits the image into work blocks and drops the remainder (src/opencl/renderer_opencl.cpp:90).
+  // The built-in pipelines render the whole image; a user's .cl kernel gets the reference's work blocks (whole image
+  // for MAX_FIT), with the remainder written as 0.
   impl->renderCommon(p->kernelFilePath, p->kernelMode, block, p->imageDimensions, p->pOutputBuffer, p->outputBufferSize,
-                    p->pAccelerationStructureExplicit, p->pModel, p->pCamera, p->pNext);
+                    p->pAccelerationStructureExplicit, p->pModel, p->pCamera, p->pNext, workBlock);
 }
