@@ -12,7 +12,8 @@
 //
 // In a round all rays are of one kind (all primary, all shadow, all extension), shading code runs on
 // dense arrays, and the running mean is applied in frame order, so results are bit-identical to
-// k_path's.  Path state lives in HBM (64 B/path) between rounds.
+// k_path's.  Between rounds a path's state travels in its queue entry, beside its ray (40 B payload), so every load
+// of a queue entry is indexed by its slot and can be issued at once.
 #include "lt_internal.h"
 #include "lt_device.cuh"
 
@@ -24,14 +25,16 @@
 #define WF_THREADED_BLOCKS_PER_SM 8  // persistent trace blocks per SM on the threaded tree
 
 struct LtWfBuffers {
-  float4* st;         // 64-byte record per path, two 32-byte sectors that are read and written independently:
-                      //   S0 = [0] nrm.xyz, -  [1] diffuse.rgb, -      (written when a surface hit is shaded)
-                      //   S1 = [2] direct.rgb, extW  [3] indirect.rgb, -   (written when a shadow result is shaded)
-                      // stage and depth travel in the queue entry's path word, hitPrim is the ray's ignore index
   float4* frameCol;   // running frame colour of the path (the 25-sample blend, or the single sample)
   float4* rayO[2];    // origin.xyz, tStart
   float4* rayD[2];    // direction.xyz, bits((ignore + 1) | anyHit << 31)
   int* rayPath[2];    // path id of the queue entry | stage << 25 | depth << 27  (WF_PATH_* below)
+  // Path state of the queue entry (WfPayload), indexed like the rays: the shade kernel loads it in queue order
+  // together with the ray and the hit instead of by path id after them.  Stage and depth travel in the path word,
+  // hitPrim is the ray's ignore index.
+  float4* payA[2];    // nrm.xyz of the shading point, then bits(material index) for a shadow ray / extW for an extension ray
+  float4* payB[2];    // direct.rgb, indirect.r
+  float2* payC[2];    // indirect.gb
   float4* hits;       // t, u, v, bits(prim | hit << 31), indexed like the current queue
   int* counts;        // [2q], [2q+1] sizes of the front and the back region of queue q (one 64-bit word per queue, so
                       // that one atomic reserves both), [4] trace work counter.  Rays that need the select-chain
@@ -68,12 +71,28 @@ __device__ __forceinline__ bool ray_is_degenerate(const Ray& r) {
   return !(finite3(FRCP(r.dx), FRCP(r.dy), FRCP(r.dz)) && finite3(r.ox, r.oy, r.oz));
 }
 
+// What the next shading of a queue entry reads of its path, beside the ray (LtWfBuffers::payA/B/C).  A shadow ray's
+// shading reads the diffuse colour of its shading point, an extension ray's the w of its direction: one word holds
+// the material index (the diffuse colour is a load from the small materials table) or extW.
+struct WfPayload {
+  float4 a, b;
+  float2 c;
+};
+
+__device__ __forceinline__ WfPayload wf_payload(const PathState& ps, float sel) {
+  WfPayload pl;
+  pl.a = make_float4(ps.nrm[0], ps.nrm[1], ps.nrm[2], sel);
+  pl.b = make_float4(ps.direct[0], ps.direct[1], ps.direct[2], ps.indirect[0]);
+  pl.c = make_float2(ps.indirect[1], ps.indirect[2]);
+  return pl;
+}
+
 // Block-aggregated append of this thread's ray (if emit) to queue `dst`; every thread of the block calls it the
 // same number of times.  One global atomic per block and call -- on a packed 64-bit counter (front count in the
 // low word, back count in the high word) -- instead of up to two per warp: ncu attributed 31 % of the shade
 // kernel's stall samples to the wait for those same-address atomics.
 __device__ __forceinline__ void queue_append(const LtWfBuffers& B, int dst, bool emit, const Ray& r, float tStart,
-                                             int ignore, bool anyHit, int path, unsigned lane) {
+                                             int ignore, bool anyHit, int path, const WfPayload& pl, unsigned lane) {
   __shared__ unsigned s_warpCount[WF_BLOCK / 32];  // front | back << 16 of each warp
   __shared__ unsigned long long s_base;
   const unsigned warp = threadIdx.x >> 5;
@@ -102,12 +121,16 @@ __device__ __forceinline__ void queue_append(const LtWfBuffers& B, int dst, bool
     B.rayD[dst][slot] = make_float4(r.dx, r.dy, r.dz,
                                     __int_as_float((int)((unsigned)(ignore + 1) | (anyHit ? 0x80000000u : 0u))));
     B.rayPath[dst][slot] = path;
+    B.payA[dst][slot] = pl.a;
+    B.payB[dst][slot] = pl.b;
+    B.payC[dst][slot] = pl.c;
   }
 }
 
 // warp-aggregated form (no block barrier) for the primary round, where most warps of a sparse view emit nothing
 __device__ __forceinline__ void queue_append_warp(const LtWfBuffers& B, int dst, bool emit, const Ray& r, float tStart,
-                                                  int ignore, bool anyHit, int path, unsigned lane) {
+                                                  int ignore, bool anyHit, int path, const WfPayload& pl,
+                                                  unsigned lane) {
   bool back = emit && ray_is_degenerate(r);
   bool front = emit && !back;
   unsigned fm = __ballot_sync(0xffffffffu, front), bm = __ballot_sync(0xffffffffu, back);
@@ -125,6 +148,9 @@ __device__ __forceinline__ void queue_append_warp(const LtWfBuffers& B, int dst,
     B.rayD[dst][slot] = make_float4(r.dx, r.dy, r.dz,
                                     __int_as_float((int)((unsigned)(ignore + 1) | (anyHit ? 0x80000000u : 0u))));
     B.rayPath[dst][slot] = path;
+    B.payA[dst][slot] = pl.a;
+    B.payB[dst][slot] = pl.b;
+    B.payC[dst][slot] = pl.c;
   }
 }
 
@@ -227,6 +253,7 @@ __global__ void __launch_bounds__(WF_BLOCK) k_wf_primary(LtSceneDev sc, LtLaunch
     float tStart = 0.0f;
     int ignore = -1, packed = 0;
     bool anyHit = false;
+    WfPayload pl = {};
     if (p < nPaths) {
       if (!STATS && P.alive != nullptr) {  // p enumerates (frame, alive pixel): turn it into the path id
         int fl = (int)(p / perFrame);
@@ -271,13 +298,11 @@ __global__ void __launch_bounds__(WF_BLOCK) k_wf_primary(LtSceneDev sc, LtLaunch
         B.frameCol[p] = make_float4(fc[0], fc[1], fc[2], 0.0f);
       } else {
         emit = true;  // a surface hit: the shadow ray of the direct light sample (direct = indirect = 0 so far)
-        float4* wr = B.st + 4ll * p;
-        wr[0] = make_float4(ps.nrm[0], ps.nrm[1], ps.nrm[2], 0.0f);
-        wr[1] = make_float4(ps.diffuse[0], ps.diffuse[1], ps.diffuse[2], 0.0f);
+        pl = wf_payload(ps, __int_as_float(sc.prims[h.prim].materialIndex));
         packed = wf_pack_path((int)p, ps.stage, ps.depth);
       }
     }
-    queue_append_warp(B, 0, emit, t.r, tStart, ignore, anyHit, packed, lane);
+    queue_append_warp(B, 0, emit, t.r, tStart, ignore, anyHit, packed, pl, lane);
   }
   if (STATS) flush_counters(gcnt, cnt);
 }
@@ -398,10 +423,13 @@ __global__ void __launch_bounds__(WF_BLOCK, 8) k_wf_shade(LtSceneDev sc, LtLaunc
     float tStart = 0.0f;
     int ignore = -1, path = 0;
     bool anyHit = false;
+    WfPayload pl = {};
     if (valid) {
       const int word = B.rayPath[q][i];
       path = word & ((1 << WF_PATH_BITS) - 1);
       float4 o = B.rayO[q][i], d = B.rayD[q][i], hv = B.hits[i];
+      const float4 pa = B.payA[q][i], pb = B.payB[q][i];
+      const float2 pc2 = B.payC[q][i];
       r.ox = o.x; r.oy = o.y; r.oz = o.z;
       r.dx = d.x; r.dy = d.y; r.dz = d.z;
       Hit h;
@@ -415,54 +443,40 @@ __global__ void __launch_bounds__(WF_BLOCK, 8) k_wf_shade(LtSceneDev sc, LtLaunc
       // every ray after the primary one ignores the primitive its path stands on (basic_lighting.cl:271,
       // global_illumination.cl:294,311,350)
       ps.hitPrim = (int)((unsigned)__float_as_int(d.w) & 0x7fffffffu) - 1;
-      // Only the half of the record this step reads is loaded:
-      //   shadow result   : nrm, diffuse (S0); the accumulators (S1) unless it is the direct sample, where they are 0
-      //   extension result: nothing for a surface hit; S0 + S1 for a light hit; S1 for a miss (final colour)
       const bool shadowStage = ps.stage == ST_SHADOW_DIRECT || ps.stage == ST_SHADOW_EXT;
       const bool lightHit = ps.stage == ST_EXTENSION && is_light(sc, h.prim);
       const bool surfaceHit = ps.stage == ST_EXTENSION && !lightHit && h.hit == 1;
-      const bool needS0 = shadowStage || lightHit;
-      const bool needS1 = ps.stage == ST_SHADOW_EXT || (ps.stage == ST_EXTENSION && !surfaceHit);
-      const float4* rec = B.st + 4ll * path;
-      float4 a = make_float4(0.0f, 0.0f, 0.0f, 0.0f), b = a, c = a, dd = a;
-      if (needS0) {
-        a = rec[0];
-        b = rec[1];
+      ps.nrm[0] = pa.x; ps.nrm[1] = pa.y; ps.nrm[2] = pa.z;
+      ps.extW = pa.w;  // read by the light hit of an extension ray only
+      ps.diffuse[0] = ps.diffuse[1] = ps.diffuse[2] = 0.0f;  // an extension result sets it or does not read it
+      if (shadowStage) {
+        const RefMaterial* mat = sc.mats + __float_as_int(pa.w);
+        ps.diffuse[0] = mat->diffuse[0]; ps.diffuse[1] = mat->diffuse[1]; ps.diffuse[2] = mat->diffuse[2];
       }
-      if (needS1) {
-        c = rec[2];
-        dd = rec[3];
-      }
-      ps.nrm[0] = a.x; ps.nrm[1] = a.y; ps.nrm[2] = a.z;
-      ps.diffuse[0] = b.x; ps.diffuse[1] = b.y; ps.diffuse[2] = b.z;
-      ps.direct[0] = c.x; ps.direct[1] = c.y; ps.direct[2] = c.z; ps.extW = c.w;
-      ps.indirect[0] = dd.x; ps.indirect[1] = dd.y; ps.indirect[2] = dd.z;
+      ps.direct[0] = pb.x; ps.direct[1] = pb.y; ps.direct[2] = pb.z;
+      ps.indirect[0] = pb.w; ps.indirect[1] = pc2.x; ps.indirect[2] = pc2.y;
       int fl;
       float fx, fy;
       film_of_path(P, path, pixels, L, fl, fx, fy);
       unsigned sampleIndex = sample_index_of(L, pc, frame0 + fl, sample);
       bool done = shade_step(sc, pc, ps, r, h, fx, fy, sampleIndex, tStart, ignore, anyHit, lightHit ? 1 : 0);
       if (done) {
-        float col[3], fc[3];
+        float col[3], fc[3] = {0.0f, 0.0f, 0.0f};
         sample_colour(pc, ps, col);
-        float4 prev = B.frameCol[path];
-        fc[0] = prev.x; fc[1] = prev.y; fc[2] = prev.z;
+        if (sample > 0) {  // blend_sample copies the first sample of a frame
+          float4 prev = B.frameCol[path];
+          fc[0] = prev.x; fc[1] = prev.y; fc[2] = prev.z;
+        }
         blend_sample(pc, sample, col, fc);
         B.frameCol[path] = make_float4(fc[0], fc[1], fc[2], 0.0f);
       } else {
         emit = true;
-        float4* wr = B.st + 4ll * path;
-        if (surfaceHit) {  // new shading point
-          wr[0] = make_float4(ps.nrm[0], ps.nrm[1], ps.nrm[2], 0.0f);
-          wr[1] = make_float4(ps.diffuse[0], ps.diffuse[1], ps.diffuse[2], 0.0f);
-        } else {  // shadow result or light hit: accumulators, w of the new extension direction
-          wr[2] = make_float4(ps.direct[0], ps.direct[1], ps.direct[2], ps.extW);
-          wr[3] = make_float4(ps.indirect[0], ps.indirect[1], ps.indirect[2], 0.0f);
-        }
+        // a surface hit is the new shading point of a shadow ray; otherwise the next ray is an extension ray
+        pl = wf_payload(ps, surfaceHit ? __int_as_float(sc.prims[h.prim].materialIndex) : ps.extW);
         path = wf_pack_path(path, ps.stage, ps.depth);
       }
     }
-    queue_append(B, 1 - q, emit, r, tStart, ignore, anyHit, path, lane);
+    queue_append(B, 1 - q, emit, r, tStart, ignore, anyHit, path, pl, lane);
   }
 }
 
@@ -503,7 +517,8 @@ __global__ void __launch_bounds__(WF_BLOCK) k_wf_accumulate(LtLaunch L, LtWfBuff
 #define LT_LAUNCH_FLAG_NO_THREADED 16  // == LT_FLAG_NO_THREADED (include/lens_trace_b200.h)
 
 size_t lt_wf_bytes_per_path() {
-  return sizeof(float4) * (4 + 1 + 2 * 2 + 1) + sizeof(int) * 2;  // state, frame colour, 2 queues, hits, path ids
+  // frame colour, hits; per queue: ray (2 x 16 B), payload (40 B), path word
+  return sizeof(float4) * 2 + 2 * (sizeof(float4) * 4 + sizeof(float2) + sizeof(int));
 }
 
 size_t lt_wf_workspace_bytes(long long nPaths) { return lt_wf_bytes_per_path() * (size_t)nPaths + 256; }
@@ -518,12 +533,14 @@ static LtWfBuffers carve(void* workspace, long long nPaths) {
   };
   B.counts = (int*)take(256);
   size_t f4 = sizeof(float4) * (size_t)nPaths;
-  B.st = (float4*)take(4 * f4);
   B.frameCol = (float4*)take(f4);
   for (int k = 0; k < 2; k++) {
     B.rayO[k] = (float4*)take(f4);
     B.rayD[k] = (float4*)take(f4);
     B.rayPath[k] = (int*)take(sizeof(int) * (size_t)nPaths);
+    B.payA[k] = (float4*)take(f4);
+    B.payB[k] = (float4*)take(f4);
+    B.payC[k] = (float2*)take(sizeof(float2) * (size_t)nPaths);
   }
   B.hits = (float4*)take(f4);
   B.capacity = (int)nPaths;
