@@ -236,6 +236,26 @@ int lt_debug_build_threaded_pruned(const void* nodes, uint64_t node_bytes, void*
  * the pruned ones.  The output is the same either way; tests compare the two. */
 int lt_debug_scene_full_threaded(lt_scene* scene, int full);
 
+/* Test hook (single-GPU contexts; LT_ERR_UNSUPPORTED on a multi-GPU one): the context's size limits.  Trees of at
+ * most threaded_max_nodes nodes (default 65536) get threaded copies built on the host at upload, larger ones copies
+ * built on the device; exact, uncounted launches of the deterministic kernels on scenes of at least stream_min_nodes
+ * nodes (default 100000) run the tile-fetching kernel.  The output is the same either way; tests lower the limits so
+ * that the small scenes the oracle can check run the large-scene paths. */
+int lt_debug_ctx_limits(lt_ctx* ctx, int threaded_max_nodes, int stream_min_nodes);
+
+/* Host-only (no device needed): the launch plan lt_render makes for `params` on a scene of node_count nodes whose
+ * traversal stack needs stack_depth levels, uploaded to a device of total_mem bytes with sm_count SMs, under the
+ * default limits; the scene has the threaded copies lt_scene_upload would make.  out receives LT_PLAN_FIELDS values:
+ *   pipeline (0 k_flat, 1 k_flat_stream, 2 k_path megakernel, 3 wavefront), tree (0 child-pair stack traversal,
+ *   1 host-built threaded copies, 2 device-built ones), stats, cull, then for the wavefront frames per batch,
+ *   streams, rounds, samples per frame, shared primary hits, pixel classification, then dynamic shared memory of the
+ *   stack-traversal kernels and of the trace kernel, blocks per SM of the persistent kernels, grid, and the wavefront
+ *   workspace bytes.
+ * Returns LT_OK, or the error lt_render would return (its message in lt_last_error(NULL)). */
+#define LT_PLAN_FIELDS 15
+int lt_debug_plan(const lt_render_params* params, uint64_t node_count, int32_t stack_depth, uint64_t total_mem,
+                  int32_t sm_count, int64_t* out);
+
 /* --- plug-in kernels: a user-written .cu file with the reference's kernel ABI (extern "C" __global__
  * linearKernel / tileKernel(LinearBVHNode*, Primitive*, Material*, LightContainer*, Camera*, float* out,
  * int width, int height, int depth), resources/kernels/cuda/basic.cu:331-340).  Replaces the NVRTC compile

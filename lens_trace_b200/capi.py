@@ -19,6 +19,7 @@ SYMBOLS = [
     "lt_scene_release", "lt_render", "lt_render_device", "lt_accum_reset", "lt_accum_read", "lt_primary_hits",
     "lt_last_stats", "lt_kernel_from_path", "lt_kernel_name", "lt_debug_random", "lt_debug_hemisphere", "lt_debug_build_threaded", "lt_debug_build_threaded_pruned", "lt_debug_scene_full_threaded", "lt_plugin_load", "lt_render_plugin", "lt_render_plugin_cl", "lt_debug_compile_cl", "lt_debug_translate_cl", "lt_primary_hits_flags", "lt_scene_build_lbvh", "lt_scene_build_ploc", "lt_scene_download", "lt_scene_info",
     "lt_debug_gather_peak", "lt_ctx_create_multi", "lt_ctx_device_count", "lt_host_register", "lt_host_unregister", "lt_debug_tile_rows",
+    "lt_debug_plan", "lt_debug_ctx_limits",
 ]
 
 
@@ -89,6 +90,9 @@ def load():
     lib.lt_debug_build_threaded.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p]
     lib.lt_debug_build_threaded_pruned.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.POINTER(C.c_int32)]
     lib.lt_debug_scene_full_threaded.argtypes = [C.c_void_p, C.c_int]
+    lib.lt_debug_ctx_limits.argtypes = [C.c_void_p, C.c_int, C.c_int]
+    lib.lt_debug_plan.argtypes = [C.POINTER(RenderParams), C.c_uint64, C.c_int32, C.c_uint64, C.c_int32,
+                                  C.POINTER(C.c_int64)]
     lib.lt_plugin_load.argtypes = [C.c_void_p, C.c_char_p, C.POINTER(C.c_int)]
     lib.lt_render_plugin.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                      C.c_int, C.c_int, C.c_void_p]
@@ -297,6 +301,11 @@ class Context:
         with finite, nonzero reciprocals walk the pruned ones again (full=False, the default after upload)."""
         self._check(self.lib.lt_debug_scene_full_threaded(scene.h, 1 if full else 0), "lt_debug_scene_full_threaded")
 
+    def debug_limits(self, threaded_max_nodes, stream_min_nodes):
+        """Test hook: trees of at most threaded_max_nodes nodes get host-built threaded copies at upload (larger ones
+        device-built copies); deterministic launches on scenes of at least stream_min_nodes nodes run k_flat_stream."""
+        self._check(self.lib.lt_debug_ctx_limits(self.h, threaded_max_nodes, stream_min_nodes), "lt_debug_ctx_limits")
+
     def stats(self):
         s = Stats()
         self.lib.lt_last_stats(self.h, C.byref(s))
@@ -322,6 +331,27 @@ def tile_rows(height, devices, device):
     out = np.zeros(n, np.int32)
     lib.lt_debug_tile_rows(height, devices, device, out.ctypes.data, n)
     return out
+
+
+PLAN_FIELDS = ("pipeline", "tree", "stats", "cull", "batch_frames", "streams", "rounds", "samples_per_frame",
+               "shared_primary", "classify", "smem_stack", "smem_trace", "blocks_per_sm", "grid", "workspace_bytes")
+PIPE_FLAT, PIPE_FLAT_STREAM, PIPE_PATH, PIPE_WAVEFRONT = range(4)
+TREE_CHILD_PAIR, TREE_HOST_THREADED, TREE_DEVICE_THREADED = range(3)
+ERR_INVALID, ERR_UNSUPPORTED = -1, -4
+
+
+def plan(params, node_count, stack_depth, total_mem, sm_count):
+    """Host-only: the launch plan lt_render makes for `params` on a scene of node_count nodes (lt_debug_plan), as a
+    dict of PLAN_FIELDS plus "error" (0 or the code lt_render returns) and "message"."""
+    lib = load()
+    out = (C.c_int64 * len(PLAN_FIELDS))()
+    rc = lib.lt_debug_plan(C.byref(params), node_count, stack_depth, total_mem, sm_count, out)
+    if rc == ERR_INVALID:
+        raise LtError("lt_debug_plan failed (%d): %s" % (rc, lib.lt_last_error(None).decode()))
+    d = dict(zip(PLAN_FIELDS, out))
+    d["error"] = rc
+    d["message"] = lib.lt_last_error(None).decode() if rc else ""
+    return d
 
 
 THREAD_NODE = np.dtype([("lo", "<f4", 3), ("hix", "<f4"), ("hiy", "<f4"), ("hiz", "<f4"), ("link", "<i4"), ("skip", "<i4")])

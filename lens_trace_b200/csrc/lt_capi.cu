@@ -108,6 +108,151 @@ int lt_internal_fail(lt_ctx* ctx, int code, const std::string& msg) { return fai
 
 int lt_internal_ctx_device(const lt_ctx* ctx) { return ctx->device; }
 
+// ------------------------------------------------------------------------------------------------
+// Launch plan: which kernels a call runs, on which tree, at which sizes.  Pure (no CUDA call, no allocation), so that
+// lt_debug_plan shows it on a machine without a GPU.
+// ------------------------------------------------------------------------------------------------
+static_assert(LT_DEV_KERNEL_BASIC_CU == LT_KERNEL_BASIC_CU && LT_DEV_KERNEL_BASIC_CL == LT_KERNEL_BASIC_CL &&
+                  LT_DEV_KERNEL_CUSTOM_BARY == LT_KERNEL_CUSTOM_BARY && LT_DEV_KERNEL_LIGHTING25 == LT_KERNEL_LIGHTING25 &&
+                  LT_DEV_KERNEL_ACCUMULATOR == LT_KERNEL_ACCUMULATOR && LT_DEV_KERNEL_GI25 == LT_KERNEL_GI25 &&
+                  LT_DEV_KERNEL_GI == LT_KERNEL_GI,
+              "lt_device_types.h: kernel ids differ from enum lt_kernel");
+static_assert(LT_DEV_FLAG_STATS == LT_FLAG_STATS && LT_DEV_FLAG_CULL == LT_FLAG_CULL &&
+                  LT_DEV_FLAG_STATS_TRACED == LT_FLAG_STATS_TRACED,
+              "lt_device_types.h: flags differ from enum lt_flags");
+
+struct LtSceneFacts {
+  int nodeCount, stackDepth;
+  LtTree copies;  // the threaded copies the scene has (LT_TREE_CHILD_PAIR: none)
+};
+
+// Threaded copies lt_scene_upload makes of a tree of nNodes nodes: built on the host up to threadedMaxNodes (8 x 32 B
+// x N for the full copies, at most as much again for the pruned ones, must stay cache resident); for larger trees the
+// full copies built on the device, unless they would not fit the budget (4 GB and an eighth of the device) or 31-bit
+// record indices.
+static LtTree lt_plan_threaded_copies(int nNodes, size_t totalMem, const LtLimits& lim) {
+  if (nNodes <= lim.threadedMaxNodes) return LT_TREE_HOST_THREADED;
+  const size_t bytes = sizeof(LtThreadNode) * 8 * (size_t)nNodes;
+  if (nNodes > 1 && bytes <= (4ull << 30) && bytes <= totalMem / 8 && (long long)nNodes * 8 < 0x7fffffffll)
+    return LT_TREE_DEVICE_THREADED;
+  return LT_TREE_CHILD_PAIR;
+}
+
+static size_t stack_smem(int stackDepth, bool cull) {  // the layout of LT_SMEM_POINTERS (lt_device.cuh)
+  return (size_t)((stackDepth < 1 ? 1 : stackDepth) * (cull ? 2 : 1) + LT_MAX_BATCH) * LT_BLOCK * sizeof(int);
+}
+
+// The threaded copies serve the exact, uncounted kernels only: the stats kernels count in the stack traversal, whose
+// tests are the same ones, the culled traversal has no threaded form, and LT_FLAG_NO_THREADED selects the stack
+// traversal for comparison.  A large scene's device-built copies serve coherent launches only (camera rays and shadow
+// rays towards a light: the two lighting kernels on the megakernel): 1 M triangles, 1080p, primary + shadow 0.96
+// instead of 1.10 ms.  For the incoherent rays of GI they lose (56.8 instead of 42.6 ms per 16-spp frame: eight copies
+// of the tree no longer fit in L2), and the tile-fetching k_flat_stream is faster on the child-pair tree (0.66 against
+// 0.72 ms: half the dependent steps per ray).
+static LtTree plan_tree(int flags, bool coherent, LtTree copies) {
+  if (flags & (LT_FLAG_STATS | LT_FLAG_CULL | LT_FLAG_NO_THREADED)) return LT_TREE_CHILD_PAIR;
+  if (copies == LT_TREE_DEVICE_THREADED && !coherent) return LT_TREE_CHILD_PAIR;
+  return copies;
+}
+
+static int tile_blocks(int width, int height) { return ((width + 15) / 16) * ((height + 7) / 8); }
+
+static LtPlan lt_plan_primary_hits(int flags, int width, int height, const LtSceneFacts& s) {
+  LtPlan p = {};
+  p.pipeline = LT_PIPE_FLAT;
+  p.tree = plan_tree(flags, false, s.copies);
+  p.cull = (flags & LT_FLAG_CULL) != 0;
+  p.smemStack = p.smemTrace = stack_smem(s.stackDepth, p.cull);
+  p.grid = tile_blocks(width, height);
+  return p;
+}
+
+static LtPlan lt_plan_render(const LtLaunch& L, const LtSceneFacts& s, size_t totalMem, int smCount,
+                             const LtLimits& lim) {
+  LtPlan p = {};
+  p.error = LT_OK;
+  p.stats = (L.flags & LT_FLAG_STATS) != 0;
+  p.cull = (L.flags & LT_FLAG_CULL) != 0;
+  const long long pixels = (long long)L.width * L.height;
+  const bool isGI = L.kernel == LT_KERNEL_GI25 || L.kernel == LT_KERNEL_GI;
+  // stochastic kernels: wavefront pipeline for large launches, persistent megakernel for small ones
+  p.pipeline = L.kernel >= LT_KERNEL_LIGHTING25 ? LT_PIPE_PATH : LT_PIPE_FLAT;
+  if (p.pipeline == LT_PIPE_PATH && !(L.flags & LT_FLAG_MEGAKERNEL)) {
+    // measured (tools/compare_pipelines.py): the wavefront wins once ~8M paths are in flight per batch; below that,
+    // and for the two-ray lighting kernels on small scenes, its per-round launches and state traffic lose.  Second
+    // measurement (shared camera rays, overlapped batches): the two-ray lighting kernels on a small scene win too
+    // once a launch holds several batches (64 frames at 1080p: 1.31x); the 25-sample kernels stay on k_path
+    const long long minPaths = 1ll << 23;
+    const long long need = (isGI || s.nodeCount > 100000) ? minPaths : 4 * minPaths;
+    const bool forced = (L.flags & (LT_FLAG_WAVEFRONT | LT_FLAG_CULL)) != 0;
+    bool wavefront = forced || (pixels * L.frames >= need && L.kernel != LT_KERNEL_GI25 &&
+                                L.kernel != LT_KERNEL_LIGHTING25);
+    // A queue entry carries the bounce depth in 5 bits (wf_pack_path): deeper bounce caps stay on the megakernel,
+    // which is the same arithmetic per path (0 = the reference constant 16).  It carries its path id in 25 bits:
+    // one frame must fit.
+    const char* unsupported = nullptr;
+    if (wavefront && isGI && L.maxRayDepth > 32)
+      unsupported = "lt_render: the wavefront pipeline handles max_ray_depth <= 32 (use the default schedule)";
+    else if (wavefront && pixels > (1ll << 25))
+      unsupported = "lt_render: the wavefront pipeline handles at most 2^25 pixels per frame";
+    if (unsupported && forced) {
+      p.error = LT_ERR_UNSUPPORTED;
+      p.message = unsupported;
+      return p;
+    }
+    if (wavefront && !unsupported) {
+      p.pipeline = LT_PIPE_WAVEFRONT;
+      p.forced = forced;
+      // paths in flight, both overlapped batches together (~200 B each), on at most 1/8 of the device
+      long long cap = 1ll << 26;
+      const long long memCap = (long long)(totalMem / 8) / 200;
+      if (cap > memCap) cap = memCap;
+      int batchFrames = (int)(cap / pixels);
+      if (batchFrames < 1) batchFrames = 1;
+      if (batchFrames > L.frames) batchFrames = L.frames;
+      // Two consecutive batches overlap on two streams (the trace kernel of one beside the shade kernel of the other:
+      // L1 data pipe vs DRAM): half-size batches, one workspace each -- same memory.  LT_FLAG_SERIAL: one stream,
+      // kernels run one at a time.  Measured: reserving room on the SMs for the other batch's blocks (fewer
+      // persistent trace blocks) does not pay, nor do 3 or 4 batches in flight (profiles/r2u_overlap_sweep.txt).
+      p.streams = !(L.flags & (LT_FLAG_SERIAL | LT_FLAG_STATS)) && L.frames >= 2 ? 2 : 1;
+      batchFrames = (batchFrames + p.streams - 1) / p.streams;
+      long long perBatch = (1ll << 25) / pixels;  // a queue entry carries its path id in 25 bits
+      if (perBatch < 1) perBatch = 1;
+      p.batchFrames = batchFrames > perBatch ? (int)perBatch : batchFrames;
+      p.samplesPerFrame = (L.kernel == LT_KERNEL_LIGHTING25 || L.kernel == LT_KERNEL_GI25) ? 25 : 1;
+      p.rounds = isGI ? 2 + 2 * (L.maxRayDepth > 0 ? L.maxRayDepth : 16) : 2;
+      p.sharedPrimary = !p.stats && !p.cull;  // the exact, uncounted pipelines
+      p.classify = p.sharedPrimary && p.samplesPerFrame == 1;
+      p.workspaceBytes = lt_wf_workspace_bytes_padded((long long)p.batchFrames * pixels) * (size_t)p.streams +
+                         lt_wf_primary_hits_bytes(pixels);
+    }
+  }
+  // camera rays and one shadow ray per hit: the two lighting kernels on the megakernel
+  const bool coherent =
+      p.pipeline == LT_PIPE_PATH && (L.kernel == LT_KERNEL_LIGHTING25 || L.kernel == LT_KERNEL_ACCUMULATOR);
+  p.tree = plan_tree(L.flags, coherent, s.copies);
+  p.smemStack = stack_smem(s.stackDepth, p.cull);
+  p.smemTrace = p.tree == LT_TREE_CHILD_PAIR ? p.smemStack : (size_t)LT_MAX_BATCH * LT_BLOCK * sizeof(int);
+  // shared memory is what limits residency of the persistent kernels (the threaded trace kernel's 8 KB: the cap of
+  // 8); k_flat_stream measured at 4 .. 10: no difference (the longest tile bounds the kernel)
+  p.blocksPerSm = (int)((200 * 1024) / p.smemTrace);
+  if (p.blocksPerSm > 8) p.blocksPerSm = 8;
+  if (p.blocksPerSm < 1) p.blocksPerSm = 1;
+  // exact, uncounted launches of the deterministic pipelines on large scenes: persistent warps fetching tiles
+  if (p.pipeline == LT_PIPE_FLAT && !(L.flags & (LT_FLAG_STATS | LT_FLAG_CULL | LT_FLAG_NO_STREAM)) &&
+      p.tree == LT_TREE_CHILD_PAIR && s.nodeCount >= lim.streamMinNodes)
+    p.pipeline = LT_PIPE_FLAT_STREAM;
+  if (p.pipeline == LT_PIPE_FLAT_STREAM) {
+    const int warpsNeeded = (((L.width + 7) >> 3) * ((L.height + 3) >> 2) + 3) / 4;  // blocks of 4 warps, one tile each
+    p.grid = smCount * p.blocksPerSm < warpsNeeded ? smCount * p.blocksPerSm : warpsNeeded;
+  } else if (p.pipeline == LT_PIPE_WAVEFRONT) {
+    p.grid = smCount * p.blocksPerSm;
+  } else {
+    p.grid = tile_blocks(L.width, L.height);
+  }
+  return p;
+}
+
 extern "C" int lt_api_version(void) { return LT_API_VERSION; }
 
 extern "C" const char* lt_last_error(const lt_ctx* ctx) { return ctx ? ctx->error.c_str() : g_error.c_str(); }
@@ -250,17 +395,7 @@ extern "C" void lt_scene_release(lt_ctx* ctx, lt_scene* s) {
 
 // Threaded form of the tree (LtThreadNode, lens_trace_b200_device.cuh): eight copies of the node array, copy o in
 // the order the reference's traversal visits the nodes for rays of sign octant o, then eight pruned copies.  Built
-// on the host: it is only made for trees of at most lt_threaded_max_nodes() nodes (8 x 32 B x N for the full copies,
-// at most as much again for the pruned ones, must stay cache resident).
-static int lt_threaded_max_nodes() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("LT_THREADED_MAX_NODES");
-    v = e ? atoi(e) : 65536;  // 16 MB of records at the limit
-    if (v < 0) v = 0;
-  }
-  return v;
-}
+// on the host, for small trees only (lt_plan_threaded_copies).
 
 // Appends eight copies of the threaded form to `out`, each in the visit order of its sign octant, leaving out the
 // nodes with keep[i] == 0.  Copy o is records [base + o * stride, base + (o + 1) * stride), base = out.size() on
@@ -437,7 +572,8 @@ static int finish_scene(lt_ctx* ctx, lt_scene* s, int nNodes, int nPrims, int nM
     lt_launch_reflatten(s->dNodes, nNodes, s->dPrims, nPrims, dRank, s->dWide, s->dTris, st);
     A(cudaGetLastError());
   }
-  if (e == cudaSuccess && nNodes <= lt_threaded_max_nodes()) {
+  const LtTree copies = lt_plan_threaded_copies(nNodes, ctx->totalMem, ctx->limits);
+  if (e == cudaSuccess && copies == LT_TREE_HOST_THREADED) {
     std::vector<RefNode> hNodes((size_t)nNodes);
     std::vector<LtThreadNode> hThread;
     A(cudaMemcpyAsync(hNodes.data(), s->dNodes, sizeof(RefNode) * (size_t)nNodes, cudaMemcpyDeviceToHost, st));
@@ -449,19 +585,14 @@ static int finish_scene(lt_ctx* ctx, lt_scene* s, int nNodes, int nPrims, int nM
       A(cudaStreamSynchronize(st));  // hThread is pageable and goes out of scope
     }
   }
-  // large trees: the threaded copies are built on the device and used by coherent-ray launches only (lt_kernels.cu:
-  // scene_for_flags); skipped when they would not fit the budget (4 GB and an eighth of the device)
-  if (e == cudaSuccess && nNodes > lt_threaded_max_nodes() && nNodes > 1) {
-    const size_t kBudget = 4ull << 30;
-    const size_t bytes = sizeof(LtThreadNode) * 8 * (size_t)nNodes;
-    if (bytes <= kBudget && bytes <= ctx->totalMem / 8 && (long long)nNodes * 8 < 0x7fffffffll) {
-      if (cudaMalloc(&s->dThreadBig, bytes) == cudaSuccess) {
-        lt_launch_build_threaded(s->dNodes, nNodes, s->dThreadBig, st);
-        A(cudaGetLastError());
-      } else {
-        cudaGetLastError();  // no memory for the copies: the stack traversal serves every launch
-        s->dThreadBig = nullptr;
-      }
+  // large trees: the threaded copies are built on the device and used by coherent-ray launches only (plan_tree)
+  if (e == cudaSuccess && copies == LT_TREE_DEVICE_THREADED) {
+    if (cudaMalloc(&s->dThreadBig, sizeof(LtThreadNode) * 8 * (size_t)nNodes) == cudaSuccess) {
+      lt_launch_build_threaded(s->dNodes, nNodes, s->dThreadBig, st);
+      A(cudaGetLastError());
+    } else {
+      cudaGetLastError();  // no memory for the copies: the stack traversal serves every launch
+      s->dThreadBig = nullptr;
     }
   }
   A(cudaEventRecord(ctx->ev1, st));
@@ -662,10 +793,8 @@ extern "C" int lt_scene_upload(lt_ctx* ctx, const void* nodes, uint64_t node_byt
   return LT_OK;
 }
 
-static int check_params(lt_ctx* ctx, const lt_scene* scene, const void* camera28, const lt_render_params* p,
-                        LtLaunch* L) {
-  if (!ctx) return fail(nullptr, LT_ERR_INVALID, "lt_render: ctx is NULL");
-  if (!scene || !camera28 || !p) return fail(ctx, LT_ERR_INVALID, "lt_render: NULL argument");
+// lt_render_params -> the launch descriptor (all of it but the camera), with lt_render's checks
+static int launch_from_params(lt_ctx* ctx, const lt_render_params* p, LtLaunch* L) {
   // API version 1 callers pass the struct without its last field (split_mode)
   if (p->struct_size != sizeof(lt_render_params) && p->struct_size != offsetof(lt_render_params, split_mode))
     return fail(ctx, LT_ERR_INVALID, "lt_render: params.struct_size mismatch");
@@ -692,7 +821,53 @@ static int check_params(lt_ctx* ctx, const lt_scene* scene, const void* camera28
   L->accumMode = p->accum_mode;
   L->accumWeight = p->accum_weight;
   L->flags = p->flags;
+  return LT_OK;
+}
+
+static int check_params(lt_ctx* ctx, const lt_scene* scene, const void* camera28, const lt_render_params* p,
+                        LtLaunch* L) {
+  if (!ctx) return fail(nullptr, LT_ERR_INVALID, "lt_render: ctx is NULL");
+  if (!scene || !camera28 || !p) return fail(ctx, LT_ERR_INVALID, "lt_render: NULL argument");
+  if (int rc = launch_from_params(ctx, p, L)) return rc;
   memcpy(&L->cam, camera28, sizeof(RefCamera));
+  return LT_OK;
+}
+
+static LtSceneFacts scene_facts(const lt_scene* s) {
+  return {s->dev.nodeCount, s->dev.stackDepth,
+          s->dThread ? LT_TREE_HOST_THREADED : (s->dThreadBig ? LT_TREE_DEVICE_THREADED : LT_TREE_CHILD_PAIR)};
+}
+
+// the scene as the plan's kernels see it: tnodes = the plan's threaded copies, NULL for the stack traversal
+static LtSceneDev scene_for_plan(const lt_scene* s, const LtPlan& plan) {
+  LtSceneDev d = s->dev;
+  d.tnodes = plan.tree == LT_TREE_HOST_THREADED ? s->dThread
+             : plan.tree == LT_TREE_DEVICE_THREADED ? s->dThreadBig : nullptr;
+  return d;
+}
+
+extern "C" int lt_debug_plan(const lt_render_params* params, uint64_t node_count, int32_t stack_depth,
+                             uint64_t total_mem, int32_t sm_count, int64_t* out) {
+  if (!params || !out || node_count < 1 || node_count > 0x7fffffffull || sm_count < 1)
+    return fail(nullptr, LT_ERR_INVALID, "lt_debug_plan: bad arguments");
+  LtLaunch L = {};
+  if (int rc = launch_from_params(nullptr, params, &L)) return rc;
+  const LtLimits lim;
+  const LtSceneFacts s = {(int)node_count, stack_depth, lt_plan_threaded_copies((int)node_count, total_mem, lim)};
+  const LtPlan p = lt_plan_render(L, s, total_mem, sm_count, lim);
+  const int64_t v[LT_PLAN_FIELDS] = {p.pipeline, p.tree, p.stats, p.cull, p.batchFrames, p.streams, p.rounds,
+                                     p.samplesPerFrame, p.sharedPrimary, p.classify, (int64_t)p.smemStack,
+                                     (int64_t)p.smemTrace, p.blocksPerSm, p.grid, (int64_t)p.workspaceBytes};
+  memcpy(out, v, sizeof v);
+  return p.error != LT_OK ? fail(nullptr, p.error, p.message) : LT_OK;
+}
+
+extern "C" int lt_debug_ctx_limits(lt_ctx* ctx, int threaded_max_nodes, int stream_min_nodes) {
+  if (!ctx) return fail(nullptr, LT_ERR_INVALID, "lt_debug_ctx_limits: ctx is NULL");
+  if (ctx->group) return fail(ctx, LT_ERR_UNSUPPORTED, "lt_debug_ctx_limits: not available on a multi-GPU context");
+  if (threaded_max_nodes < 0 || stream_min_nodes < 0) return fail(ctx, LT_ERR_INVALID, "lt_debug_ctx_limits: negative limit");
+  ctx->limits.threadedMaxNodes = threaded_max_nodes;
+  ctx->limits.streamMinNodes = stream_min_nodes;
   return LT_OK;
 }
 
@@ -711,71 +886,26 @@ int lt_internal_ensure_out(lt_ctx* ctx, size_t floats) {
 
 static int render_common(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, float* dOut, bool sync) {
   CK(cudaSetDevice(ctx->device));
-  bool stats = (L.flags & LT_FLAG_STATS) != 0;
+  LtPlan plan = lt_plan_render(L, scene_facts(scene), ctx->totalMem, ctx->stats.sm_count, ctx->limits);
+  if (plan.error != LT_OK) return fail(ctx, plan.error, plan.message);
+  const bool stats = plan.stats;
   if (stats) CK(cudaMemsetAsync(ctx->dCounters, 0, sizeof(LtCounters), ctx->stream));
-  // stochastic kernels: wavefront pipeline for large launches, persistent megakernel for small ones
-  bool wavefront = false, overlapBatches = false;
-  int batchFrames = 1;
-  if (L.kernel >= 3 && !(L.flags & LT_FLAG_MEGAKERNEL)) {
-    long long pixels = (long long)L.width * L.height;
-    const long long minPaths = 1ll << 23;
-    // paths in flight, both overlapped batches together (~200 B each); a queue entry carries its path id in 25 bits
-    const long long maxPaths = 1ll << 26;
-    // measured (tools/compare_pipelines.py): the wavefront wins once ~8M paths are in flight per batch; below
-    // that, and for the two-ray lighting kernels on small scenes, its per-round launches and state traffic lose
-    bool isGI = (L.kernel == 5 || L.kernel == 6);
-    bool bigScene = scene->dev.nodeCount > 100000;
-    // second measurement (shared camera rays, overlapped batches): the two-ray lighting kernels on a small scene win
-    // too once a launch holds several batches (64 frames at 1080p: 1.31x); the 25-sample kernels stay on k_path
-    long long need = (isGI || bigScene) ? minPaths : 4 * minPaths;
-    wavefront = (L.flags & (LT_FLAG_WAVEFRONT | LT_FLAG_CULL)) ||
-                (pixels * L.frames >= need && L.kernel != 5 && L.kernel != 3);
-    // a queue entry carries the bounce depth in 5 bits (wf_pack_path): deeper bounce caps stay on the megakernel,
-    // which is the same arithmetic per path (0 = the reference constant 16)
-    if (wavefront && isGI && L.maxRayDepth > 32) {
-      if (L.flags & (LT_FLAG_WAVEFRONT | LT_FLAG_CULL))
-        return fail(ctx, LT_ERR_UNSUPPORTED, "lt_render: the wavefront pipeline handles max_ray_depth <= 32 (use the default schedule)");
-      wavefront = false;
-    }
-    if (wavefront && pixels > (1ll << 25)) {  // a queue entry carries its path id in 25 bits: one frame must fit
-      if (L.flags & (LT_FLAG_WAVEFRONT | LT_FLAG_CULL))
-        return fail(ctx, LT_ERR_UNSUPPORTED, "lt_render: the wavefront pipeline handles at most 2^25 pixels per frame");
-      wavefront = false;
-    }
-    if (wavefront) {
-      long long cap = maxPaths;
-      long long memCap = (long long)(ctx->totalMem / 8) / 200;  // at most 1/8 of the device for the workspace
-      if (cap > memCap) cap = memCap;
-      batchFrames = (int)(cap / pixels);
-      if (batchFrames < 1) batchFrames = 1;
-      if (batchFrames > L.frames) batchFrames = L.frames;
-      // two consecutive batches overlap on two streams (trace of one beside shade of the other): half-size batches,
-      // one workspace each -- same memory.  LT_FLAG_SERIAL: one stream, kernels run one at a time.
-      overlapBatches = !(L.flags & (LT_FLAG_SERIAL | LT_FLAG_STATS)) && L.frames >= 2;
-      const int nStreams = overlapBatches ? 2 : 1;
-      batchFrames = (batchFrames + nStreams - 1) / nStreams;
-      {  // a queue entry carries its path id in 25 bits: at most 2^25 paths per batch
-        long long perBatch = (1ll << 25) / pixels;
-        if (perBatch < 1) perBatch = 1;
-        if (batchFrames > perBatch) batchFrames = (int)perBatch;
-      }
-      size_t need = lt_wf_workspace_bytes_padded((long long)batchFrames * pixels) * (size_t)nStreams +
-                    lt_wf_primary_hits_bytes(pixels);
-      if (ctx->wfBytes < need) {
-        if (ctx->wfWorkspace) cudaFree(ctx->wfWorkspace);
-        ctx->wfWorkspace = nullptr;
-        ctx->wfBytes = 0;
-        if (cudaMalloc(&ctx->wfWorkspace, need) != cudaSuccess) {
-          cudaGetLastError();
-          if (L.flags & (LT_FLAG_WAVEFRONT | LT_FLAG_CULL))
-            return fail(ctx, LT_ERR_CUDA, "lt_render: cannot allocate the wavefront workspace");
-          wavefront = false;  // not a fallback to other arithmetic: the megakernel is the same path per pixel
-        } else {
-          ctx->wfBytes = need;
-        }
-      }
+  if (plan.pipeline == LT_PIPE_WAVEFRONT && ctx->wfBytes < plan.workspaceBytes) {
+    if (ctx->wfWorkspace) cudaFree(ctx->wfWorkspace);
+    ctx->wfWorkspace = nullptr;
+    ctx->wfBytes = 0;
+    if (cudaMalloc(&ctx->wfWorkspace, plan.workspaceBytes) != cudaSuccess) {
+      cudaGetLastError();
+      if (plan.forced) return fail(ctx, LT_ERR_CUDA, "lt_render: cannot allocate the wavefront workspace");
+      // not a fallback to other arithmetic: the megakernel is the same path per pixel
+      LtLaunch mega = L;
+      mega.flags |= LT_FLAG_MEGAKERNEL;
+      plan = lt_plan_render(mega, scene_facts(scene), ctx->totalMem, ctx->stats.sm_count, ctx->limits);
+    } else {
+      ctx->wfBytes = plan.workspaceBytes;
     }
   }
+  const bool wavefront = plan.pipeline == LT_PIPE_WAVEFRONT;
   const int kMaxTracePairs = 8192;
   int tracePairs = 0;
   bool timeTrace = wavefront && (sync || stats);
@@ -785,15 +915,15 @@ static int render_common(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, float*
     for (size_t i = 0; i < ctx->traceEvents.size(); i++) cudaEventCreate(&ctx->traceEvents[i]);
   }
   // per-kernel times are only defined when one kernel runs at a time (LT_FLAG_SERIAL / stats launches)
-  const bool timeKinds = timeTrace && (!overlapBatches);
+  const bool timeKinds = timeTrace && plan.streams == 1;
+  const LtSceneDev sc = scene_for_plan(scene, plan);
   CK(cudaEventRecord(ctx->ev0, ctx->stream));
-  int launches = wavefront ? lt_launch_render_wavefront(scene->dev, L, dOut, ctx->dCounters, ctx->wfWorkspace,
-                                                        batchFrames, ctx->stats.sm_count, ctx->stream,
+  int launches = wavefront ? lt_launch_render_wavefront(sc, plan, L, dOut, ctx->dCounters, ctx->wfWorkspace,
+                                                        ctx->stats.sm_count, ctx->stream,
                                                         timeTrace ? ctx->traceEvents.data() : nullptr, kMaxTracePairs,
                                                         &tracePairs, timeKinds ? ctx->pairKinds.data() : nullptr,
-                                                        overlapBatches ? &ctx->wfAux : nullptr)
-                           : lt_launch_render(scene->dev, L, dOut, ctx->dCounters, ctx->dWork, ctx->stats.sm_count,
-                                              ctx->stream);
+                                                        &ctx->wfAux)
+                           : lt_launch_render(sc, plan, L, dOut, ctx->dCounters, ctx->dWork, ctx->stream);
   CK(cudaGetLastError());
   CK(cudaEventRecord(ctx->ev1, ctx->stream));
   ctx->stats.kernel_launches = launches;
@@ -1125,7 +1255,9 @@ static int primary_hits_impl(lt_ctx* ctx, lt_scene* scene, const void* camera28,
   float* dTuv = reinterpret_cast<float*>(dAll + 2 * n);
   RefCamera cam;
   memcpy(&cam, camera28, sizeof(cam));
-  lt_launch_primary_hits(scene->dev, cam, kernel, flags, width, height, dIds, dHit, dTuv, ctx->stream);
+  const LtPlan plan = lt_plan_primary_hits(flags, width, height, scene_facts(scene));
+  lt_launch_primary_hits(scene_for_plan(scene, plan), plan, cam, kernel, flags, width, height, dIds, dHit, dTuv,
+                         ctx->stream);
   cudaError_t e = cudaGetLastError();
   if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
   if (e == cudaSuccess && ids) e = cudaMemcpy(ids, dIds, n * sizeof(int), cudaMemcpyDeviceToHost);
@@ -1180,7 +1312,7 @@ static const char* kKernelNames[LT_KERNEL_COUNT] = {"basic.cu",       "basic.cl"
                                                     "global_illumination.cl(1)"};
 
 extern "C" const char* lt_kernel_name(int kernel) {
-  return (kernel >= 0 && kernel < LT_KERNEL_COUNT) ? kKernelNames[kernel] : "unknown";
+  return (kernel < 0 || kernel >= LT_KERNEL_COUNT) ? "unknown" : kKernelNames[kernel];
 }
 
 // kernelFilePath -> built-in pipeline, by CONTENT (the reference compiles whatever text the file holds,

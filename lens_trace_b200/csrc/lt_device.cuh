@@ -13,7 +13,6 @@
 #endif
 #endif
 
-#define LT_BLOCK 128
 // Per-thread stacks and leaf FIFOs live in shared memory as [level][thread]: LT_THREAD_STRIDE ints between the levels
 // of one thread.  The library's kernels run blocks of LT_BLOCK threads; a plug-in build (any block shape) defines
 // the stride as its run-time block size before including this file.
@@ -251,8 +250,8 @@ __device__ __forceinline__ void trav_node_step(Trav& t, const LtSceneDev& sc, in
 // so box tests and triangle tests are decoupled: the node phase walks the tree and only RECORDS the
 // leaves it reaches, in order, in a small per-thread list in shared memory; the leaf phase then
 // tests the recorded triangles in that order.  A warp therefore switches between "all lanes test
-// boxes" and "all lanes test triangles" once per batch instead of at every leaf.
-#define LT_MAX_BATCH 16  // list entries per thread (shared memory: [LT_MAX_BATCH][LT_BLOCK] ints)
+// boxes" and "all lanes test triangles" once per batch instead of at every leaf.  The list holds LT_MAX_BATCH
+// entries (lt_device_types.h).
 
 // node phase: advance until the ray is exhausted (t.cur == LT_DONE) or `batch` leaves are recorded.
 // Returns the number of recorded leaves.
@@ -582,13 +581,8 @@ __device__ __forceinline__ void trace_cull(Trav& t, const LtSceneDev& sc, int ig
 }
 
 // dynamic shared memory of every traversal kernel: [stackDepth][LT_BLOCK] stack, [LT_MAX_BATCH][LT_BLOCK] leaf
-// list/FIFO, [stackDepth][LT_BLOCK] entry distances (culled mode only)
+// list/FIFO, [stackDepth][LT_BLOCK] entry distances (culled mode only); lt_capi.cu: stack_smem sizes it
 __host__ __device__ inline int lt_stack_levels(const LtSceneDev& sc) { return sc.stackDepth < 1 ? 1 : sc.stackDepth; }
-#ifndef __CUDACC_RTC__
-__host__ inline size_t lt_traversal_smem(const LtSceneDev& sc, bool cull) {
-  return (size_t)(lt_stack_levels(sc) * (cull ? 2 : 1) + LT_MAX_BATCH) * LT_BLOCK * sizeof(int);
-}
-#endif
 #define LT_SMEM_POINTERS(sc)                                                            \
   extern __shared__ int smemStack[];                                                    \
   int* stk = smemStack + threadIdx.x;                                                   \
@@ -616,12 +610,13 @@ __device__ __forceinline__ void trace(Trav& t, const LtSceneDev& sc, int ignore,
 // ------------------------------------------------------------------------------------------------
 // per-kernel constants (see oracle/lt_oracle.c: flavour_for_kernel)
 // ------------------------------------------------------------------------------------------------
-__host__ __device__ inline float lt_tinit(int kernel) { return kernel == 0 ? 10000000.0f : FLT_MAX; }
+__host__ __device__ inline float lt_tinit(int kernel) { return kernel == LT_DEV_KERNEL_BASIC_CU ? 10000000.0f : FLT_MAX; }
 __host__ __device__ inline float lt_eps(int kernel) {
   // fabs(det) < eps; the macro-defined epsilons are compared in fp64, i.e. against the next float up
   switch (kernel) {
-    case 0: case 1: case 2: return 0x1.ad7f2ap-24f;  // (float)1e-7: basic.cu:95, basic.cl:78
-    case 3: return 0x1.ad7f2ap-24f;                   // (float)1e-7 >= 1e-7 (double) already
+    case LT_DEV_KERNEL_BASIC_CU: case LT_DEV_KERNEL_BASIC_CL: case LT_DEV_KERNEL_CUSTOM_BARY:
+      return 0x1.ad7f2ap-24f;  // (float)1e-7: basic.cu:95, basic.cl:78
+    case LT_DEV_KERNEL_LIGHTING25: return 0x1.ad7f2ap-24f;  // (float)1e-7 >= 1e-7 (double) already
     default: return 0x1.a36e30p-14f;                  // smallest float >= 1e-4 (double); (float)1e-4 is below
   }
 }
@@ -911,13 +906,13 @@ __device__ __forceinline__ PathConsts path_consts(const LtLaunch& L) {
   PathConsts pc;
   pc.tInit = lt_tinit(L.kernel);
   pc.epsThr = lt_eps(L.kernel);
-  pc.isGI = (L.kernel == 5 || L.kernel == 6);
-  pc.whiteOnLight = (L.kernel == 4);
-  pc.samplesPerFrame = (L.kernel == 3 || L.kernel == 5) ? 25 : 1;
+  pc.isGI = (L.kernel == LT_DEV_KERNEL_GI25 || L.kernel == LT_DEV_KERNEL_GI);
+  pc.whiteOnLight = (L.kernel == LT_DEV_KERNEL_ACCUMULATOR);
+  pc.samplesPerFrame = (L.kernel == LT_DEV_KERNEL_LIGHTING25 || L.kernel == LT_DEV_KERNEL_GI25) ? 25 : 1;
   pc.maxDepth = L.maxRayDepth > 0 ? L.maxRayDepth : 16;
-  // counting launches (LT_FLAG_STATS = 1) trace what the reference traces, unless LT_FLAG_STATS_TRACED = 128 asks for
-  // the counts of what the exact pipelines really trace
-  pc.foldLightHits = !(L.flags & 1) || (L.flags & 128);
+  // counting launches trace what the reference traces, unless LT_FLAG_STATS_TRACED asks for the counts of what the
+  // exact pipelines really trace
+  pc.foldLightHits = !(L.flags & LT_DEV_FLAG_STATS) || (L.flags & LT_DEV_FLAG_STATS_TRACED);
   return pc;
 }
 

@@ -3,6 +3,22 @@
 #pragma once
 #include "lens_trace_b200_device.cuh"  // buffer layouts
 
+// The values of enum lt_kernel and enum lt_flags (include/lens_trace_b200.h) that the device code tests: NVRTC cannot
+// include the public header.  lt_capi.cu checks that both agree.
+constexpr int LT_DEV_KERNEL_BASIC_CU = 0;
+constexpr int LT_DEV_KERNEL_BASIC_CL = 1;
+constexpr int LT_DEV_KERNEL_CUSTOM_BARY = 2;
+constexpr int LT_DEV_KERNEL_LIGHTING25 = 3;
+constexpr int LT_DEV_KERNEL_ACCUMULATOR = 4;
+constexpr int LT_DEV_KERNEL_GI25 = 5;
+constexpr int LT_DEV_KERNEL_GI = 6;
+constexpr int LT_DEV_FLAG_STATS = 1 << 0;
+constexpr int LT_DEV_FLAG_CULL = 1 << 1;
+constexpr int LT_DEV_FLAG_STATS_TRACED = 1 << 7;
+
+#define LT_BLOCK 128     // threads per block of the library's traversal kernels
+#define LT_MAX_BATCH 16  // leaf-list entries per thread (shared memory: [LT_MAX_BATCH][LT_BLOCK] ints)
+
 struct LtLaunch {
   int kernel;        // lt_kernel
   int kernelMode;    // 0 linear, 1 tile

@@ -11,7 +11,36 @@
 struct lt_ctx;
 int lt_internal_ctx_device(const lt_ctx* ctx);  // lt_capi.cu
 
-// launchers implemented in lt_kernels.cu (all asynchronous on `stream`; return launches made)
+// ---- launch plan (lt_capi.cu: lt_plan_render): every choice of which kernels run, on which tree, at which sizes ----
+// k_flat, k_flat_stream, k_path, or the wavefront pipeline (lt_wavefront.cu)
+enum LtPipeline { LT_PIPE_FLAT, LT_PIPE_FLAT_STREAM, LT_PIPE_PATH, LT_PIPE_WAVEFRONT };
+// the tree the traversal kernels walk: child-pair nodes with a stack, or the host- or device-built threaded copies
+enum LtTree { LT_TREE_CHILD_PAIR, LT_TREE_HOST_THREADED, LT_TREE_DEVICE_THREADED };
+// Per-context limits of the plan and of the upload-time layout; lt_debug_ctx_limits changes them for tests.
+struct LtLimits {
+  int threadedMaxNodes = 65536;  // trees up to this size get host-built threaded copies (16 MB of records at the limit)
+  int streamMinNodes = 100000;   // deterministic kernels on scenes this large: k_flat_stream
+};
+struct LtPlan {
+  int error;            // LT_OK, or what lt_render returns (with `message`)
+  const char* message;
+  LtPipeline pipeline;
+  LtTree tree;
+  bool stats, cull;
+  bool forced;          // the caller asked for the wavefront: no megakernel in its place when its workspace fails
+  // wavefront only
+  int batchFrames, streams, rounds, samplesPerFrame;
+  bool sharedPrimary;   // camera rays traced once per pixel for all frames of the launch
+  bool classify;        // ... and pixels without paths (background, light) skipped
+  size_t workspaceBytes;
+  // dynamic shared memory of the stack-traversal kernels, and of the trace kernel (threaded or stack)
+  size_t smemStack, smemTrace;
+  int blocksPerSm;      // persistent kernels (k_flat_stream, k_wf_trace)
+  int grid;             // blocks: persistent grid, or one block per 16x8 tile (k_flat, k_path)
+};
+
+// launchers implemented in lt_kernels.cu (all asynchronous on `stream`; return launches made).  The launchers of the
+// traversal kernels take the scene with the plan's tree in `tnodes`.
 int lt_launch_reflatten(const RefNode* dNodes, int nodeCount, const RefPrim* dPrims, int primCount,
                         const int* dInnerRank, LtWideNode* dWide, LtTri* dTris, cudaStream_t stream);
 int lt_launch_inner_flags(const RefNode* dNodes, int nodeCount, int* dFlags, cudaStream_t stream);
@@ -19,10 +48,14 @@ int lt_launch_build_threaded(const RefNode* dNodes, int nodeCount, LtThreadNode*
 size_t lt_scan_temp_bytes(int n);
 int lt_launch_exclusive_scan(void* dTemp, size_t tempBytes, const int* dIn, int* dOut, int n, cudaStream_t stream);
 // dWork: one zero-initialisable int of device memory (work counter of the persistent kernels)
-int lt_launch_render(const LtSceneDev& sc, const LtLaunch& L, float* dOut, LtCounters* dCounters, int* dWork,
-                     int smCount, cudaStream_t stream);
-int lt_launch_primary_hits(const LtSceneDev& sc, const RefCamera& cam, int kernel, int flags, int width, int height,
-                           int* dIds, int* dHit, float* dTuv, cudaStream_t stream);
+int lt_launch_render(const LtSceneDev& sc, const LtPlan& plan, const LtLaunch& L, float* dOut, LtCounters* dCounters,
+                     int* dWork, cudaStream_t stream);
+int lt_launch_primary_hits(const LtSceneDev& sc, const LtPlan& plan, const RefCamera& cam, int kernel, int flags,
+                           int width, int height, int* dIds, int* dHit, float* dTuv, cudaStream_t stream);
+// Dynamic shared memory beyond 48 KB needs an opt-in per kernel and device: given once for every traversal kernel
+// (both files), the first time a launch asks for more.
+void lt_opt_in_traversal_smem(size_t smem);
+extern const void* const lt_wf_traversal_kernels[5];  // lt_wavefront.cu
 int lt_launch_debug_random(const float* fx, const float* fy, const float* seed, int n, float* out, cudaStream_t stream);
 int lt_launch_debug_hemisphere(const float* u1, const float* u2, const float* up, int n, float* out,
                                cudaStream_t stream);
@@ -32,10 +65,10 @@ size_t lt_wf_workspace_bytes_padded(long long nPaths);
 size_t lt_wf_primary_hits_bytes(long long pixels);  // per-launch primary hit records, kept behind the batch workspaces
 // traceEvents: optional pool of 2*maxTraceLaunches events; when given, every traversal launch is bracketed by a
 // pair of events and *traceLaunches receives the number of pairs recorded
-// aux: a second stream + events (fork, one batch-order event per stream) for overlapping consecutive batches (the
-// L1-bound trace kernel of one batch runs beside the DRAM-bound shade kernel of the other and fills the tail of the
-// persistent kernels); `workspace` then holds two batch workspaces of
-// lt_wf_workspace_bytes_padded(batchFrames * pixels) each.  aux == nullptr: one stream.
+// aux: a second stream + events (fork, one batch-order event per stream), used when the plan overlaps consecutive
+// batches on two streams (the L1-bound trace kernel of one batch runs beside the DRAM-bound shade kernel of the other
+// and fills the tail of the persistent kernels); `workspace` then holds two batch workspaces of
+// lt_wf_workspace_bytes_padded(batchFrames * pixels) each.
 struct LtWfAux {
   cudaStream_t extra;  // odd batches; even batches run on the caller's stream
   cudaEvent_t fork, order[2];
@@ -43,8 +76,8 @@ struct LtWfAux {
 // pairKinds: optional, one LT_TIMED_* per recorded pair; when given, the shade / primary-shade / accumulate launches
 // are bracketed as well (per-kernel times of a serialised step)
 enum { LT_TIMED_TRAVERSAL = 0, LT_TIMED_SHADE = 1, LT_TIMED_PRIMARY_SHADE = 2, LT_TIMED_ACCUMULATE = 3, LT_TIMED_KINDS = 4 };
-int lt_launch_render_wavefront(const LtSceneDev& sc, const LtLaunch& L, float* dOut, LtCounters* dCounters,
-                               void* workspace, int batchFrames, int smCount, cudaStream_t stream,
+int lt_launch_render_wavefront(const LtSceneDev& sc, const LtPlan& plan, const LtLaunch& L, float* dOut,
+                               LtCounters* dCounters, void* workspace, int smCount, cudaStream_t stream,
                                cudaEvent_t* traceEvents, int maxTraceLaunches, int* traceLaunches,
                                unsigned char* pairKinds, const LtWfAux* aux);
 
@@ -97,6 +130,7 @@ struct lt_ctx {
   size_t stageBytes = 0;
   std::vector<cudaEvent_t> stageEvents;  // one per 2 MB chunk
   LtCopyPool* copyPool = nullptr;
+  LtLimits limits;
   lt_stats stats = {};
 };
 

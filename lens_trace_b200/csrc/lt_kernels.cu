@@ -18,9 +18,6 @@
 #include "lt_device.cuh"
 
 #include <cub/device/device_scan.cuh>
-#include <stdlib.h>
-
-#define LT_LAUNCH_FLAG_NO_STREAM 64  // == LT_FLAG_NO_STREAM (include/lens_trace_b200.h)
 
 template <bool STATS>
 __global__ void __launch_bounds__(LT_BLOCK) k_flat(LtSceneDev sc, LtLaunch L, float* __restrict__ out,
@@ -34,11 +31,11 @@ __global__ void __launch_bounds__(LT_BLOCK) k_flat(LtSceneDev sc, LtLaunch L, fl
   t.r = camera_ray(L.cam, px, lt_image_row(L, py), L.width, L.fullHeight, fx, fy);
   const float tInit = lt_tinit(L.kernel), epsThr = lt_eps(L.kernel);
   float color[3] = {0.0f, 0.0f, 0.0f};
-  const bool cull = (L.flags & 2) != 0;  // LT_FLAG_CULL
+  const bool cull = (L.flags & LT_DEV_FLAG_CULL) != 0;
   if (cull) trace_cull<STATS>(t, sc, -1, tInit, epsThr, stk, tstk, cnt);
   else trace<STATS>(t, sc, -1, tInit, epsThr, false, stk, list, cnt);
   if (t.h.hit == 1) {
-    if (L.kernel == 2) {  // custom_opencl.cl:240
+    if (L.kernel == LT_DEV_KERNEL_CUSTOM_BARY) {  // custom_opencl.cl:240
       color[0] = t.h.u;
       color[1] = t.h.v;
       color[2] = bary0(t.h.u, t.h.v);
@@ -112,7 +109,7 @@ __global__ void __launch_bounds__(LT_BLOCK) k_flat_stream(LtSceneDev sc, LtLaunc
       const Hit h = t.h;
       if (stage == 0) {
         if (h.hit != 1) break;
-        if (L.kernel == 2) {  // custom_opencl.cl:240
+        if (L.kernel == LT_DEV_KERNEL_CUSTOM_BARY) {  // custom_opencl.cl:240
           color[0] = h.u;
           color[1] = h.v;
           color[2] = bary0(h.u, h.v);
@@ -127,7 +124,7 @@ __global__ void __launch_bounds__(LT_BLOCK) k_flat_stream(LtSceneDev sc, LtLaunc
         baseMat = sc.prims[h.prim].materialIndex;
       }
     }
-    if (L.kernel != 2 && (t.h.hit == 1 || ignore >= 0)) {
+    if (L.kernel != LT_DEV_KERNEL_CUSTOM_BARY && (t.h.hit == 1 || ignore >= 0)) {
       const RefMaterial* mat = sc.mats + baseMat;
       color[0] = mat->diffuse[0];
       color[1] = mat->diffuse[1];
@@ -265,7 +262,7 @@ __global__ void __launch_bounds__(LT_BLOCK) k_primary_hits(LtSceneDev sc, RefCam
   float fx, fy;
   Trav t;
   t.r = camera_ray(cam, px, py, width, height, fx, fy);
-  if (flags & 2) trace_cull<false>(t, sc, -1, lt_tinit(kernel), lt_eps(kernel), stk, tstk, cnt);
+  if (flags & LT_DEV_FLAG_CULL) trace_cull<false>(t, sc, -1, lt_tinit(kernel), lt_eps(kernel), stk, tstk, cnt);
   else trace<false>(t, sc, -1, lt_tinit(kernel), lt_eps(kernel), false, stk, list, cnt);
   const Hit h = t.h;
   long long i = (long long)py * width + px;
@@ -421,85 +418,43 @@ int lt_launch_reflatten(const RefNode* dNodes, int nodeCount, const RefPrim* dPr
   return 2;
 }
 
-static size_t stack_bytes(const LtSceneDev& sc, bool cull) { return lt_traversal_smem(sc, cull); }
-
-// Dynamic shared memory beyond 48 KB needs an opt-in per kernel (and per device): the culled mode on a tree deeper
-// than 40 levels asks for up to (2 * 64 + 16) * 512 = 73 728 bytes.
+// The culled mode on a tree deeper than 40 levels asks for up to (2 * 64 + 16) * 512 = 73 728 bytes.
 #define LT_MAX_TRAVERSAL_SMEM ((2 * 64 + LT_MAX_BATCH) * LT_BLOCK * (int)sizeof(int))
-static void opt_in_smem(size_t smem) {
+void lt_opt_in_traversal_smem(size_t smem) {
   if (smem <= 48 * 1024) return;
   static bool done[64] = {};
   int dev = 0;
   cudaGetDevice(&dev);
   if (dev < 0 || dev >= 64 || done[dev]) return;
   done[dev] = true;
-  cudaFuncSetAttribute(k_flat<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, LT_MAX_TRAVERSAL_SMEM);
-  cudaFuncSetAttribute(k_flat<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, LT_MAX_TRAVERSAL_SMEM);
-  cudaFuncSetAttribute(k_path<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, LT_MAX_TRAVERSAL_SMEM);
-  cudaFuncSetAttribute(k_path<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, LT_MAX_TRAVERSAL_SMEM);
-  cudaFuncSetAttribute(k_primary_hits, cudaFuncAttributeMaxDynamicSharedMemorySize, LT_MAX_TRAVERSAL_SMEM);
-  cudaFuncSetAttribute(k_flat_stream, cudaFuncAttributeMaxDynamicSharedMemorySize, LT_MAX_TRAVERSAL_SMEM);
+  const void* const mine[] = {(const void*)k_flat<false>, (const void*)k_flat<true>, (const void*)k_path<false>,
+                              (const void*)k_path<true>, (const void*)k_primary_hits, (const void*)k_flat_stream};
+  for (const void* k : mine) cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, LT_MAX_TRAVERSAL_SMEM);
+  for (const void* k : lt_wf_traversal_kernels)
+    cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, LT_MAX_TRAVERSAL_SMEM);
 }
 
-static int tile_blocks(int width, int height) { return ((width + 15) / 16) * ((height + 7) / 8); }
-
-// the threaded tree is used by the exact, uncounted kernels only (the stats kernels count in the stack traversal,
-// whose tests are the same ones; LT_FLAG_NO_THREADED = 16 selects the stack traversal for comparison)
-// coherent: the launch traces camera rays and shadow rays towards a light only (the two lighting kernels on the
-// megakernel) -- a large scene's threaded copies (tnodesCoherent) then pay: 1 M triangles, 1080p, primary + shadow
-// 0.96 instead of 1.10 ms.  For the incoherent rays of GI they lose (56.8 instead of 42.6 ms per 16-spp frame: eight
-// copies of the tree no longer fit in L2), and the tile-fetching k_flat_stream is faster on the child-pair tree
-// (0.66 against 0.72 ms: half the dependent steps per ray)
-static LtSceneDev scene_for_flags(const LtSceneDev& sc, int flags, bool coherent = false) {
-  LtSceneDev s = sc;
-  if (coherent && s.tnodes == nullptr) s.tnodes = s.tnodesCoherent;
-  if (flags & (1 | 2 | 16)) s.tnodes = nullptr;
-  return s;
-}
-
-static int env_int(const char* name, int dflt) {
-  const char* e = getenv(name);
-  return e ? atoi(e) : dflt;
-}
-
-int lt_launch_render(const LtSceneDev& scIn, const LtLaunch& L, float* dOut, LtCounters* dCounters, int* dWork,
-                     int smCount, cudaStream_t stream) {
-  // camera rays and one shadow ray per hit: the two lighting kernels
-  const bool coherentRays = L.kernel == 3 || L.kernel == 4;
-  const LtSceneDev sc = scene_for_flags(scIn, L.flags, coherentRays);
-  int blocks = tile_blocks(L.width, L.height);
-  size_t smem = stack_bytes(sc, (L.flags & 2) != 0);
-  opt_in_smem(smem);
-  bool stats = (L.flags & 1) != 0;
-  bool flat = (L.kernel <= 2);
-  // exact, uncounted launches of the deterministic pipelines on large scenes: persistent warps fetching tiles
-  if (flat && !(L.flags & (1 | 2 | LT_LAUNCH_FLAG_NO_STREAM)) && dWork != nullptr && sc.tnodes == nullptr &&
-      sc.nodeCount >= env_int("LT_STREAM_MIN_NODES", 100000)) {
-    int blocksPerSm = (int)((200 * 1024) / smem);
-    if (blocksPerSm > 8) blocksPerSm = 8;  // measured 4 .. 10: no difference (the longest tile bounds the kernel)
-    if (blocksPerSm < 1) blocksPerSm = 1;
-    int grid = smCount * blocksPerSm;
-    const int warpsNeeded = (((L.width + 7) >> 3) * ((L.height + 3) >> 2) + 3) / 4;  // blocks of 4 warps, one tile each
-    if (grid > warpsNeeded) grid = warpsNeeded;
+int lt_launch_render(const LtSceneDev& sc, const LtPlan& plan, const LtLaunch& L, float* dOut, LtCounters* dCounters,
+                     int* dWork, cudaStream_t stream) {
+  lt_opt_in_traversal_smem(plan.smemStack);
+  const size_t smem = plan.smemStack;
+  if (plan.pipeline == LT_PIPE_FLAT_STREAM) {
     cudaMemsetAsync(dWork, 0, sizeof(int), stream);
-    k_flat_stream<<<grid, LT_BLOCK, smem, stream>>>(sc, L, dOut, dWork);
-    return 1;
-  }
-  if (flat) {
-    if (stats) k_flat<true><<<blocks, LT_BLOCK, smem, stream>>>(sc, L, dOut, dCounters);
-    else k_flat<false><<<blocks, LT_BLOCK, smem, stream>>>(sc, L, dOut, nullptr);
+    k_flat_stream<<<plan.grid, LT_BLOCK, smem, stream>>>(sc, L, dOut, dWork);
+  } else if (plan.pipeline == LT_PIPE_FLAT) {
+    if (plan.stats) k_flat<true><<<plan.grid, LT_BLOCK, smem, stream>>>(sc, L, dOut, dCounters);
+    else k_flat<false><<<plan.grid, LT_BLOCK, smem, stream>>>(sc, L, dOut, nullptr);
   } else {
-    if (stats) k_path<true><<<blocks, LT_BLOCK, smem, stream>>>(sc, L, dOut, dCounters);
-    else k_path<false><<<blocks, LT_BLOCK, smem, stream>>>(sc, L, dOut, nullptr);
+    if (plan.stats) k_path<true><<<plan.grid, LT_BLOCK, smem, stream>>>(sc, L, dOut, dCounters);
+    else k_path<false><<<plan.grid, LT_BLOCK, smem, stream>>>(sc, L, dOut, nullptr);
   }
   return 1;
 }
 
-int lt_launch_primary_hits(const LtSceneDev& scIn, const RefCamera& cam, int kernel, int flags, int width, int height,
-                           int* dIds, int* dHit, float* dTuv, cudaStream_t stream) {
-  const LtSceneDev sc = scene_for_flags(scIn, flags);
-  opt_in_smem(stack_bytes(sc, (flags & 2) != 0));
-  k_primary_hits<<<tile_blocks(width, height), LT_BLOCK, stack_bytes(sc, (flags & 2) != 0), stream>>>(
-      sc, cam, kernel, flags, width, height, dIds, dHit, dTuv);
+int lt_launch_primary_hits(const LtSceneDev& sc, const LtPlan& plan, const RefCamera& cam, int kernel, int flags,
+                           int width, int height, int* dIds, int* dHit, float* dTuv, cudaStream_t stream) {
+  lt_opt_in_traversal_smem(plan.smemStack);
+  k_primary_hits<<<plan.grid, LT_BLOCK, plan.smemStack, stream>>>(sc, cam, kernel, flags, width, height, dIds, dHit,
+                                                                   dTuv);
   return 1;
 }

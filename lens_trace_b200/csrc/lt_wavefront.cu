@@ -22,7 +22,6 @@
 // idle lanes a warp waits for before it fetches new rays: lanes that start together walk the top of the tree
 // together and share its cache lines (measured: 8 is ~1 % faster than 1 on both the 83-node and the 2 M-node tree)
 #define WF_REFILL_LANES 8
-#define WF_THREADED_BLOCKS_PER_SM 8  // persistent trace blocks per SM on the threaded tree
 
 struct LtWfBuffers {
   float4* frameCol;   // running frame colour of the path (the 25-sample blend, or the single sample)
@@ -238,7 +237,7 @@ __global__ void __launch_bounds__(WF_BLOCK) k_wf_primary(LtSceneDev sc, LtLaunch
                                                          int pixels, int sample, LtCounters* gcnt, LtWfPrimary P) {
   LT_SMEM_POINTERS(sc)
   const float4* __restrict__ primaryHits = P.hits;
-  const bool cull = (L.flags & 2) != 0;  // LT_FLAG_CULL: closest-hit rays skip subtrees behind the current hit
+  const bool cull = (L.flags & LT_DEV_FLAG_CULL) != 0;  // closest-hit rays skip subtrees behind the current hit
   const PathConsts pc = path_consts(L);
   const unsigned lane = threadIdx.x & 31u;
   LtCounters cnt = {0, 0, 0};
@@ -326,7 +325,7 @@ __global__ void __launch_bounds__(WF_BLOCK) __maxnreg__(STATS ? 64 : 56)
   int* stk = smemStack + threadIdx.x;
   int* list = smemStack + (THREADED ? 0 : lt_stack_levels(sc) * LT_BLOCK) + threadIdx.x;
   float* tstk = reinterpret_cast<float*>(smemStack + (lt_stack_levels(sc) + LT_MAX_BATCH) * LT_BLOCK) + threadIdx.x;
-  const bool cull = !THREADED && (L.flags & 2) != 0;  // LT_FLAG_CULL: closest-hit rays skip subtrees behind the current hit
+  const bool cull = !THREADED && (L.flags & LT_DEV_FLAG_CULL) != 0;  // closest-hit rays skip subtrees behind the current hit
   const int nFront = B.counts[2 * q];
   const int n = nFront + B.counts[2 * q + 1];  // virtual entries: front region, then the back region
   const float epsThr = lt_eps(L.kernel);
@@ -514,8 +513,6 @@ __global__ void __launch_bounds__(WF_BLOCK) k_wf_accumulate(LtLaunch L, LtWfBuff
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
-#define LT_LAUNCH_FLAG_NO_THREADED 16  // == LT_FLAG_NO_THREADED (include/lens_trace_b200.h)
-
 size_t lt_wf_bytes_per_path() {
   // frame colour, hits; per queue: ray (2 x 16 B), payload (40 B), path word
   return sizeof(float4) * 2 + 2 * (sizeof(float4) * 4 + sizeof(float2) + sizeof(int));
@@ -559,12 +556,15 @@ size_t lt_wf_primary_hits_bytes(long long pixels) {
   return (sizeof(float4) + sizeof(float2) + sizeof(int) + 1) * (size_t)pixels + 1024 + 5 * 256;  // 5 arrays, 256-aligned
 }
 
-int lt_launch_render_wavefront(const LtSceneDev& scIn, const LtLaunch& L, float* dOut, LtCounters* dCounters,
-                               void* workspace, int batchFrames, int smCount, cudaStream_t stream,
+// the kernels whose shared memory grows with the stack depth (lt_opt_in_traversal_smem)
+const void* const lt_wf_traversal_kernels[5] = {
+    (const void*)k_wf_primary_trace, (const void*)k_wf_primary<false>, (const void*)k_wf_primary<true>,
+    (const void*)k_wf_trace<false, false>, (const void*)k_wf_trace<true, false>};
+
+int lt_launch_render_wavefront(const LtSceneDev& sc, const LtPlan& plan, const LtLaunch& L, float* dOut,
+                               LtCounters* dCounters, void* workspace, int smCount, cudaStream_t stream,
                                cudaEvent_t* traceEvents, int maxTraceLaunches, int* traceLaunches,
                                unsigned char* pairKinds, const LtWfAux* aux) {
-  LtSceneDev sc = scIn;
-  if (L.flags & (1 | 2 | LT_LAUNCH_FLAG_NO_THREADED)) sc.tnodes = nullptr;  // stats / culled / forced stack traversal
   int pairs = 0;
   // which: 0 = before, 1 = after a launch; kind (LT_TIMED_*): what the bracketed kernel does.  Traversal launches
   // are always bracketed when events are given, the other kinds only when the caller passes pairKinds.
@@ -577,47 +577,17 @@ int lt_launch_render_wavefront(const LtSceneDev& scIn, const LtLaunch& L, float*
       pairs++;
     }
   };
+  lt_opt_in_traversal_smem(plan.smemStack);
   const int pixels = L.width * L.height;
-  const bool stats = (L.flags & 1) != 0;
-  const bool isGI = (L.kernel == 5 || L.kernel == 6);
-  const int samples = (L.kernel == 3 || L.kernel == 5) ? 25 : 1;
-  const int maxDepth = L.maxRayDepth > 0 ? L.maxRayDepth : 16;
-  const int rounds = isGI ? 2 + 2 * maxDepth : 2;
-  const size_t smem = lt_traversal_smem(sc, (L.flags & 2) != 0);
-  if (smem > 48 * 1024) {  // beyond 48 KB (culled mode on a tree deeper than 40) dynamic shared memory is an opt-in
-    static bool done[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev >= 0 && dev < 64 && !done[dev]) {
-      done[dev] = true;
-      const int most = (2 * 64 + LT_MAX_BATCH) * LT_BLOCK * (int)sizeof(int);
-      cudaFuncSetAttribute(k_wf_primary_trace, cudaFuncAttributeMaxDynamicSharedMemorySize, most);
-      cudaFuncSetAttribute(k_wf_primary<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, most);
-      cudaFuncSetAttribute(k_wf_primary<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, most);
-      cudaFuncSetAttribute(k_wf_trace<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, most);
-      cudaFuncSetAttribute(k_wf_trace<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, most);
-    }
-  }
-  int blocksPerSm = (int)((200 * 1024) / smem);  // shared memory is what limits residency of the persistent kernel
-  if (blocksPerSm > 8) blocksPerSm = 8;
-  if (blocksPerSm < 1) blocksPerSm = 1;
-  // small scenes: stackless traversal of the threaded tree (exact mode only; the stats variant counts in the
-  // stack kernel, whose tests are the same ones)
-  const bool threaded = sc.tnodes != nullptr;
-  const size_t smemTrace = threaded ? (size_t)LT_MAX_BATCH * LT_BLOCK * sizeof(int) : smem;
-  if (threaded) blocksPerSm = WF_THREADED_BLOCKS_PER_SM;
-  // Two batches in flight on two streams: the trace kernel of one batch runs beside the shade kernel of the other
-  // (different bottlenecks: L1 data pipe vs DRAM).  Measured: reserving room on the SMs for the other batch's blocks
-  // (fewer persistent trace blocks) does not pay, nor do 3 or 4 batches in flight (profiles/r2u_overlap_sweep.txt).
-  const bool overlap = aux != nullptr && L.frames > batchFrames;
-  const int nStreams = overlap ? 2 : 1;
-  const int persistentBlocks = smCount * blocksPerSm;
+  const bool stats = plan.stats, threaded = plan.tree != LT_TREE_CHILD_PAIR, overlap = plan.streams == 2;
+  const int batchFrames = plan.batchFrames;
+  const size_t smem = plan.smemStack;
   const size_t wsBytes = lt_wf_workspace_bytes_padded((long long)batchFrames * pixels);
   int preLaunches = 0;
-  // primary hits once per pixel per launch (exact, uncounted pipelines); kept behind the batch workspaces
+  // primary hits once per pixel per launch; kept behind the batch workspaces
   LtWfPrimary P = {};
-  if (!stats && !(L.flags & 2)) {
-    char* pb = (char*)workspace + (size_t)nStreams * wsBytes;  // 256-aligned: wsBytes is a multiple of 256
+  if (plan.sharedPrimary) {
+    char* pb = (char*)workspace + (size_t)plan.streams * wsBytes;  // 256-aligned: wsBytes is a multiple of 256
     auto take = [&](size_t bytes) {
       char* r = pb;
       pb += (bytes + 255) & ~(size_t)255;
@@ -629,15 +599,15 @@ int lt_launch_render_wavefront(const LtSceneDev& scIn, const LtLaunch& L, float*
     while ((1ll << l) < pixels) l++;
     P.divS = 25 + l;
     P.divM = (unsigned long long)(((1ull << P.divS) + (unsigned long long)pixels - 1ull) / (unsigned long long)pixels);
-    const bool classify = samples == 1;
-    if (classify) {
+    if (plan.classify) {
       P.alive = (int*)take(sizeof(int) * (size_t)pixels);
       P.aliveCount = (int*)take(256);
       P.cls = (unsigned char*)take((size_t)pixels);
       cudaMemsetAsync(P.aliveCount, 0, sizeof(int), stream);
     }
     mark(0, stream);
-    k_wf_primary_trace<<<(pixels + WF_BLOCK - 1) / WF_BLOCK, WF_BLOCK, smem, stream>>>(sc, L, P, pixels, classify ? 1 : 0);
+    k_wf_primary_trace<<<(pixels + WF_BLOCK - 1) / WF_BLOCK, WF_BLOCK, smem, stream>>>(sc, L, P, pixels,
+                                                                                         plan.classify ? 1 : 0);
     mark(1, stream);
     preLaunches = 1;
   }
@@ -657,7 +627,7 @@ int lt_launch_render_wavefront(const LtSceneDev& scIn, const LtLaunch& L, float*
     Lb.cam.frameCount = L.cam.frameCount + (unsigned)frame0 * L.frameStride;  // frame index 0 of the batch
     int grid = (int)((nPaths + WF_BLOCK - 1) / WF_BLOCK);
     if (grid > smCount * 32) grid = smCount * 32;
-    for (int s = 0; s < samples; s++) {
+    for (int s = 0; s < plan.samplesPerFrame; s++) {
       // round 0 (primary rays) fused into one kernel; its survivors are queue 0
       k_wf_reset<<<1, 1, 0, st>>>(B);
       // a traversal kernel only when it traces the camera rays itself
@@ -667,11 +637,11 @@ int lt_launch_render_wavefront(const LtSceneDev& scIn, const LtLaunch& L, float*
       mark(1, st, primaryHits ? LT_TIMED_PRIMARY_SHADE : LT_TIMED_TRAVERSAL);
       launches += 2;
       int q = 0;
-      for (int r = 1; r < rounds; r++) {
+      for (int r = 1; r < plan.rounds; r++) {
         mark(0, st);
-        if (stats) k_wf_trace<true, false><<<persistentBlocks, WF_BLOCK, smem, st>>>(sc, Lb, B, q, dCounters, B.rayO[q], B.rayD[q]);
-        else if (threaded) k_wf_trace<false, true><<<persistentBlocks, WF_BLOCK, smemTrace, st>>>(sc, Lb, B, q, nullptr, B.rayO[q], B.rayD[q]);
-        else k_wf_trace<false, false><<<persistentBlocks, WF_BLOCK, smem, st>>>(sc, Lb, B, q, nullptr, B.rayO[q], B.rayD[q]);
+        if (stats) k_wf_trace<true, false><<<plan.grid, WF_BLOCK, smem, st>>>(sc, Lb, B, q, dCounters, B.rayO[q], B.rayD[q]);
+        else if (threaded) k_wf_trace<false, true><<<plan.grid, WF_BLOCK, plan.smemTrace, st>>>(sc, Lb, B, q, nullptr, B.rayO[q], B.rayD[q]);
+        else k_wf_trace<false, false><<<plan.grid, WF_BLOCK, smem, st>>>(sc, Lb, B, q, nullptr, B.rayO[q], B.rayD[q]);
         mark(1, st);
         mark(0, st, LT_TIMED_SHADE);
         if (q == 0) k_wf_shade<0><<<grid, WF_BLOCK, 0, st>>>(sc, Lb, B, pixels, 0, s, P);

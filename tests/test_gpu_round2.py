@@ -165,10 +165,12 @@ def test_unreachable_nodes_are_rejected(ctx):
 # ---------------------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("name", ["green_wall", "cornell_box", "cornell_box_lens"])
 @pytest.mark.parametrize("size", [(1920, 1080), (257, 130), (7, 3), (1, 1)])
-def test_streamed_flat_kernel_equals_one_thread_per_pixel(ctx, name, size, monkeypatch):
+def test_streamed_flat_kernel_equals_one_thread_per_pixel(name, size):
     """k_flat_stream (persistent warps that fetch 8x4 tiles; the default on large scenes, forced here on the small
-    ones through LT_STREAM_MIN_NODES=0) == k_flat == the oracle, including the lens path and the frame combiner."""
-    monkeypatch.setenv("LT_STREAM_MIN_NODES", "0")
+    ones through a context whose stream_min_nodes limit is 0) == k_flat == the oracle, including the lens path and the
+    frame combiner."""
+    ctx = capi.Context(0)
+    ctx.debug_limits(threaded_max_nodes=65536, stream_min_nodes=0)
     sb = util.scene(name)
     sc = ctx.upload(sb)
     w, h = size
@@ -188,6 +190,7 @@ def test_streamed_flat_kernel_equals_one_thread_per_pixel(ctx, name, size, monke
                                              flags=L.FLAG_NO_STREAM))
     util.assert_bit_equal(a[..., :3], b[..., :3], "running mean of a deterministic kernel")
     sc.release()
+    ctx.close()
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -236,9 +239,9 @@ def test_synth1m_shadow_and_gi_all_schedules(ctx, synth1m):
 
 
 def test_synth1m_4k_five_frames(ctx, synth1m):
-    """3840x2160, 5 frames on the 1 M-triangle mesh: 8.3 M pixels per frame -> four frames per wavefront batch
-    (path ids are 25 bits), two overlapped batches.  Whole frame: wavefront == megakernel bit for bit; bands == the
-    oracle's running mean of the same five frames."""
+    """3840x2160, 5 frames on the 1 M-triangle mesh: 8.3 M pixels per frame -> three frames per wavefront batch
+    (path ids are 25 bits: at most four; five frames halved for two overlapped batches).  Whole frame: wavefront ==
+    megakernel bit for bit; bands == the oracle's running mean of the same five frames."""
     sb, sc = synth1m
     w, h, frames = 3840, 2160, 5
     cam0 = util.default_camera(0.0, 0)
@@ -311,36 +314,25 @@ def test_sah_tree_on_the_gpu(ctx, tmp_path):
         sc.release()
 
 
-def test_device_built_threaded_copies(root):
+def test_device_built_threaded_copies():
     """Large trees get their eight threaded (skip-pointer) copies from a device kernel (k_build_threaded) and use them
-    for coherent-ray launches.  LT_THREADED_MAX_NODES=0 (read once per process, hence the subprocess) sends the small
-    test scenes down that path too: deterministic and lighting kernels must still equal the oracle bit for bit, and the
-    records must equal the host-built ones the small scenes normally use."""
-    import subprocess
-    import sys
-    code = r'''
-import sys
-sys.path[:0] = [%r, %r + "/oracle", %r + "/tests"]
-import numpy as np
-import lt_oracle as O, util
-from lens_trace_b200 import capi, layouts as L
-ctx = capi.Context(0)
-for name in ("cornell_box", "cornell_box_lens", "green_wall", "single"):
-    sb = util.single_triangle_scene() if name == "single" else util.scene(name)
-    sc = ctx.upload(sb)
-    for yaw in (0.0, 0.05, -2.5):
-        cam = util.default_camera(yaw, 2)
-        for kernel in (L.KERNEL_BASIC_CU, L.KERNEL_CUSTOM_BARY, L.KERNEL_ACCUMULATOR, L.KERNEL_LIGHTING25):
-            w, h = (160, 100) if kernel != L.KERNEL_LIGHTING25 else (48, 32)
-            got = ctx.render(sc, cam, capi.make_params(kernel, w, h, flags=L.FLAG_MEGAKERNEL if kernel >= 3 else 0))
-            want = O.render(kernel, sb, cam, w, h, threads=0)
-            bad = (got.view(np.uint32) != want.view(np.uint32)).any(axis=-1).sum()
-            assert bad <= (3 if kernel >= 3 else 0), (name, yaw, kernel, int(bad))
-            stack = ctx.render(sc, cam, capi.make_params(kernel, w, h, flags=L.FLAG_NO_THREADED | (L.FLAG_MEGAKERNEL if kernel >= 3 else 0)))
-            assert (got.view(np.uint32) == stack.view(np.uint32)).all(), (name, yaw, kernel)
-    sc.release()
-print("ok")
-''' % (root, root, root)
-    env = dict(os.environ, LT_THREADED_MAX_NODES="0", LT_STREAM_MIN_NODES="0")
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600, env=env)
-    assert r.returncode == 0 and "ok" in r.stdout, r.stdout + r.stderr
+    for coherent-ray launches.  A context whose threaded_max_nodes limit is 0 sends the small test scenes down that
+    path too: deterministic and lighting kernels must still equal the oracle bit for bit, and the stack traversal."""
+    ctx = capi.Context(0)
+    ctx.debug_limits(threaded_max_nodes=0, stream_min_nodes=0)
+    for name in ("cornell_box", "cornell_box_lens", "green_wall", "single"):
+        sb = util.single_triangle_scene() if name == "single" else util.scene(name)
+        sc = ctx.upload(sb)
+        for yaw in (0.0, 0.05, -2.5):
+            cam = util.default_camera(yaw, 2)
+            for kernel in (L.KERNEL_BASIC_CU, L.KERNEL_CUSTOM_BARY, L.KERNEL_ACCUMULATOR, L.KERNEL_LIGHTING25):
+                w, h = (160, 100) if kernel != L.KERNEL_LIGHTING25 else (48, 32)
+                mega = L.FLAG_MEGAKERNEL if kernel >= L.KERNEL_LIGHTING25 else 0
+                got = ctx.render(sc, cam, capi.make_params(kernel, w, h, flags=mega))
+                want = O.render(kernel, sb, cam, w, h, threads=0)
+                bad = (got.view(np.uint32) != want.view(np.uint32)).any(axis=-1).sum()
+                assert bad <= (3 if kernel >= L.KERNEL_LIGHTING25 else 0), (name, yaw, kernel, int(bad))
+                stack = ctx.render(sc, cam, capi.make_params(kernel, w, h, flags=L.FLAG_NO_THREADED | mega))
+                assert (got.view(np.uint32) == stack.view(np.uint32)).all(), (name, yaw, kernel)
+        sc.release()
+    ctx.close()
