@@ -3,8 +3,11 @@
 //   samples : GPU g renders frames g, g+G, ...; one NCCL all-reduce of the accumulators per call
 //   tiles   : GPU g renders every G-th block of 8 image rows; no collective
 // Prints the wall time of the call per device count and the largest difference from the one-GPU picture.
+// --kernel names another kernel file: a user's own .cl or .cu file is compiled once and rendered by every GPU (sample
+// split only; the file sets its own bounce count, --depth applies to the built-in kernel).
 //
-//   bin/multi_gpu [--devices N] [--size W H] [--frames F] [--depth D] [--split samples|tiles] [--model obj] [--out file.pfm]
+//   bin/multi_gpu [--devices N] [--size W H] [--frames F] [--depth D] [--split samples|tiles] [--model obj]
+//                 [--kernel file] [--out file.pfm]
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
@@ -25,6 +28,7 @@ int main(int argc, char** argv) {
   uint32_t frames = 64, depth = 4, devices = 2, split = 1;
   const char* modelPath = "resources/models/cornell_box.obj";
   const char* outName = NULL;
+  const char* kernelPath = "examples/global_illumination/resources/kernels/global_illumination.cl";
   for (int i = 1; i < argc; i++) {
     if (!strcmp(argv[i], "--size") && i + 2 < argc) { width = strtoull(argv[++i], NULL, 10); height = strtoull(argv[++i], NULL, 10); }
     else if (!strcmp(argv[i], "--frames") && i + 1 < argc) frames = (uint32_t)atoi(argv[++i]);
@@ -33,6 +37,7 @@ int main(int argc, char** argv) {
     else if (!strcmp(argv[i], "--split") && i + 1 < argc) split = !strcmp(argv[++i], "tiles") ? 2u : 1u;
     else if (!strcmp(argv[i], "--model") && i + 1 < argc) modelPath = argv[++i];
     else if (!strcmp(argv[i], "--out") && i + 1 < argc) outName = argv[++i];
+    else if (!strcmp(argv[i], "--kernel") && i + 1 < argc) kernelPath = argv[++i];
   }
   Camera camera(0, 2.5, -50, 0);
   Model model(modelPath);
@@ -52,7 +57,7 @@ int main(int argc, char** argv) {
   RenderPropertiesOpenCL props = {};
   props.sType = STRUCTURE_TYPE_RENDER_PROPERTIES_OPENCL;
   props.pNext = &ext;
-  props.kernelFilePath = "examples/global_illumination/resources/kernels/global_illumination.cl";
+  props.kernelFilePath = kernelPath;
   props.kernelMode = KERNEL_MODE_LINEAR;
   props.threadOrganizationMode = THREAD_ORGANIZATION_MODE_MAX_FIT;
   props.imageDimensions[0] = width;
@@ -82,8 +87,8 @@ int main(int argc, char** argv) {
     if (d > maxRel) maxRel = d;
     if (one[i] != many[i]) differing++;
   }
-  printf("%llux%llu, %u frames, %u bounces, split = %s\n", (unsigned long long)width, (unsigned long long)height, frames,
-         depth, split == 2 ? "tiles" : "samples");
+  printf("%s\n%llux%llu, %u frames, %u bounces, split = %s\n", kernelPath, (unsigned long long)width,
+         (unsigned long long)height, frames, depth, split == 2 ? "tiles" : "samples");
   printf("1 GPU : %.2f ms per call\n%u GPUs: %.2f ms per call (%.2fx)\n", ms[0], devices, ms[1], ms[0] / ms[1]);
   printf("largest relative difference from the one-GPU picture: %.3g (%zu of %zu floats differ)\n", maxRel, differing,
          one.size());

@@ -444,7 +444,8 @@ private:
   uint64_t useCounter;
   uint64_t seenRetireGeneration;
   std::map<std::string, int> kernelCache;
-  std::map<std::string, int> pluginCache;  // user .cu kernels compiled for this context
+  std::map<std::string, int> pluginCache;  // user .cu / .cl kernels compiled for this context
+  std::map<std::string, int> groupPluginCache;  // ... and for groupCtx
 
 public:
   RendererB200();

@@ -260,8 +260,10 @@ int lt_debug_plan(const lt_render_params* params, uint64_t node_count, int32_t s
  * linearKernel / tileKernel(LinearBVHNode*, Primitive*, Material*, LightContainer*, Camera*, float* out,
  * int width, int height, int depth), resources/kernels/cuda/basic.cu:331-340).  Replaces the NVRTC compile
  * and launch of src/cuda/renderer_cuda.cpp:20-39,57-88,113-133 for files that are not one of the shipped
- * kernels: compiled once per context for sm_100a, then launched on the scene's buffers in the reference
- * layouts with the reference's launch shape (block_x x block_y threads, 32x1 when 0). --- */
+ * kernels: compiled once per context for sm_100a (once for all devices of a multi-GPU context, which loads it on
+ * each), then launched on the scene's buffers in the reference layouts with the reference's launch shape
+ * (block_x x block_y threads, 32x1 when 0).  lt_render_plugin and lt_render_plugin_cl render one frame on a
+ * single-GPU context (LT_ERR_UNSUPPORTED on a multi-GPU one); lt_render_plugin_frames renders many, on either. --- */
 int lt_plugin_load(lt_ctx* ctx, const char* kernel_file_path, int* out_plugin_id);
 int lt_render_plugin(lt_ctx* ctx, lt_scene* scene, const void* camera28, int plugin_id, int kernel_mode, int width,
                      int height, int depth, int block_x, int block_y, float* host_out);
@@ -285,6 +287,20 @@ int lt_render_plugin(lt_ctx* ctx, lt_scene* scene, const void* camera28, int plu
 int lt_render_plugin_cl(lt_ctx* ctx, lt_scene* scene, const void* camera28, int plugin_id, int kernel_mode, int width,
                         int height, int depth, int work_block_x, int work_block_y, int group_x, int group_y,
                         float* host_out);
+/* A plug-in (lt_plugin_load) rendered like lt_render renders a built-in kernel: params->frames frames, frame k with
+ * camera frameCount + k * frame_stride, combined by params->accum_mode into the context's accumulator (the one lt_render,
+ * lt_accum_reset and lt_accum_read use), divided among the devices of a multi-GPU context by the sample split.
+ * work_block_x/y: .cl plug-ins only (as lt_render_plugin_cl; nonzero for a .cu plug-in is LT_ERR_INVALID);
+ * params->block_x/y is the CUDA block of a .cu plug-in and the work-group of a .cl plug-in.  params->kernel and
+ * max_ray_depth are ignored (a plug-in has its own bounce cap), as are the schedule flags; LT_FLAG_STATS,
+ * LT_FLAG_STATS_TRACED and LT_FLAG_CULL return LT_ERR_UNSUPPORTED.  LT_ACCUM_NONE launches every frame into the output
+ * in order, like consecutive lt_render_plugin calls; the accumulating modes launch every frame into a sample buffer
+ * and fold it into the accumulator with the built-in pipelines' arithmetic (one extra kernel per frame).  A .cl
+ * plug-in's uncovered pixels read 0.  On a multi-GPU context: LT_SPLIT_AUTO means samples, LT_SPLIT_TILES and
+ * LT_ACCUM_NONE return LT_ERR_UNSUPPORTED, a running mean needs frame_stride 1.  Synchronous; lt_stats.kernel_ms
+ * covers the call, kernel_launches counts the plug-in and fold launches, the counters are 0. */
+int lt_render_plugin_frames(lt_ctx* ctx, lt_scene* scene, const void* camera28, int plugin_id,
+                            const lt_render_params* params, int work_block_x, int work_block_y, float* host_out);
 /* Host-only (NVRTC, no device or driver needed): translate and compile a .cl file as lt_plugin_load would.  Returns 0,
  * or LT_ERR_UNSUPPORTED with the reason / NVRTC log copied into log (NUL-terminated, truncated to log_bytes). */
 int lt_debug_compile_cl(const char* kernel_file_path, char* log, uint64_t log_bytes);

@@ -19,7 +19,7 @@ SYMBOLS = [
     "lt_scene_release", "lt_render", "lt_render_device", "lt_accum_reset", "lt_accum_read", "lt_primary_hits",
     "lt_last_stats", "lt_kernel_from_path", "lt_kernel_name", "lt_debug_random", "lt_debug_hemisphere", "lt_debug_build_threaded", "lt_debug_build_threaded_pruned", "lt_debug_scene_full_threaded", "lt_plugin_load", "lt_render_plugin", "lt_render_plugin_cl", "lt_debug_compile_cl", "lt_debug_translate_cl", "lt_primary_hits_flags", "lt_scene_build_lbvh", "lt_scene_build_ploc", "lt_scene_download", "lt_scene_info",
     "lt_debug_gather_peak", "lt_ctx_create_multi", "lt_ctx_device_count", "lt_host_register", "lt_host_unregister", "lt_debug_tile_rows",
-    "lt_debug_plan", "lt_debug_ctx_limits",
+    "lt_debug_plan", "lt_debug_ctx_limits", "lt_render_plugin_frames",
 ]
 
 
@@ -97,6 +97,8 @@ def load():
     lib.lt_render_plugin.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                      C.c_int, C.c_int, C.c_void_p]
     lib.lt_render_plugin_cl.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p] + [C.c_int] * 9 + [C.c_void_p]
+    lib.lt_render_plugin_frames.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(RenderParams), C.c_int,
+                                            C.c_int, C.c_void_p]
     lib.lt_debug_compile_cl.argtypes = [C.c_char_p, C.c_char_p, C.c_uint64]
     lib.lt_debug_translate_cl.argtypes = [C.c_char_p, C.c_char_p, C.c_uint64, C.POINTER(C.c_int32)]
     lib.lt_debug_translate_cl.restype = C.c_int64
@@ -273,6 +275,18 @@ class Context:
         self._check(self.lib.lt_render_plugin_cl(self.h, scene.h, cam.ctypes.data, plugin_id, kernel_mode, width, height,
                                                  depth, work_block[0], work_block[1], group[0], group[1],
                                                  out.ctypes.data), "lt_render_plugin_cl")
+        return out
+
+    def render_plugin_frames(self, scene, camera, plugin_id, params, work_block=(0, 0), want_output=True):
+        """params.frames frames of a plug-in combined by params.accum_mode (lt_render_plugin_frames), on one device or
+        divided among the devices of a multi-device Context.  params.block_x/y: the CUDA block of a .cu plug-in, the
+        work-group of a .cl plug-in; work_block: .cl plug-ins only.  Returns float32 [H, W, depth] or None."""
+        out = np.empty((params.height, params.width, params.depth), dtype=np.float32) if want_output else None
+        cam = np.ascontiguousarray(camera, dtype=L.CAMERA)
+        self._check(self.lib.lt_render_plugin_frames(self.h, scene.h, cam.ctypes.data, plugin_id, C.byref(params),
+                                                     work_block[0], work_block[1],
+                                                     out.ctypes.data if out is not None else None),
+                    "lt_render_plugin_frames")
         return out
 
     def debug_random(self, fx, fy, seed):

@@ -313,6 +313,7 @@ extern "C" void lt_ctx_destroy(lt_ctx* ctx) {
   if (ctx->dWork) cudaFree(ctx->dWork);
   if (ctx->wfWorkspace) cudaFree(ctx->wfWorkspace);
   if (ctx->dCamera) cudaFree(ctx->dCamera);
+  if (ctx->dSample) cudaFree(ctx->dSample);
   delete ctx->copyPool;
   if (ctx->stage) cudaFreeHost(ctx->stage);
   for (cudaEvent_t e : ctx->stageEvents) cudaEventDestroy(e);
@@ -793,19 +794,21 @@ extern "C" int lt_scene_upload(lt_ctx* ctx, const void* nodes, uint64_t node_byt
   return LT_OK;
 }
 
-// lt_render_params -> the launch descriptor (all of it but the camera), with lt_render's checks
-static int launch_from_params(lt_ctx* ctx, const lt_render_params* p, LtLaunch* L) {
+// lt_render_params -> the launch descriptor (all of it but the camera), with lt_render's checks; `who` names the entry
+// point in error messages
+static int launch_from_params(lt_ctx* ctx, const lt_render_params* p, LtLaunch* L, const char* who = "lt_render") {
+  const std::string w = std::string(who) + ": ";
   // API version 1 callers pass the struct without its last field (split_mode)
   if (p->struct_size != sizeof(lt_render_params) && p->struct_size != offsetof(lt_render_params, split_mode))
-    return fail(ctx, LT_ERR_INVALID, "lt_render: params.struct_size mismatch");
-  if (p->kernel < 0 || p->kernel >= LT_KERNEL_COUNT) return fail(ctx, LT_ERR_UNSUPPORTED, "lt_render: unknown kernel id");
+    return fail(ctx, LT_ERR_INVALID, w + "params.struct_size mismatch");
+  if (p->kernel < 0 || p->kernel >= LT_KERNEL_COUNT) return fail(ctx, LT_ERR_UNSUPPORTED, w + "unknown kernel id");
   if (p->width <= 0 || p->height <= 0 || p->depth < 3)
-    return fail(ctx, LT_ERR_INVALID, "lt_render: width/height must be > 0 and depth >= 3");
-  if ((long long)p->width * p->height * p->depth > (1ll << 40)) return fail(ctx, LT_ERR_INVALID, "lt_render: image too large");
-  if (p->frames < 1) return fail(ctx, LT_ERR_INVALID, "lt_render: frames must be >= 1");
-  if (p->accum_mode < 0 || p->accum_mode > 2) return fail(ctx, LT_ERR_INVALID, "lt_render: bad accum_mode");
+    return fail(ctx, LT_ERR_INVALID, w + "width/height must be > 0 and depth >= 3");
+  if ((long long)p->width * p->height * p->depth > (1ll << 40)) return fail(ctx, LT_ERR_INVALID, w + "image too large");
+  if (p->frames < 1) return fail(ctx, LT_ERR_INVALID, w + "frames must be >= 1");
+  if (p->accum_mode < 0 || p->accum_mode > 2) return fail(ctx, LT_ERR_INVALID, w + "bad accum_mode");
   if (p->max_ray_depth < 0 || p->max_ray_depth > 255)
-    return fail(ctx, LT_ERR_INVALID, "lt_render: max_ray_depth must be in [0, 255]");
+    return fail(ctx, LT_ERR_INVALID, w + "max_ray_depth must be in [0, 255]");
   L->kernel = p->kernel;
   L->kernelMode = p->kernel_mode ? 1 : 0;
   L->width = p->width;
@@ -1067,7 +1070,7 @@ int lt_internal_download(lt_ctx* ctx, float* host_out, const float* dSrc, size_t
 
 extern "C" int lt_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params,
                          float* host_out) {
-  if (ctx && ctx->group) return lt_multi_render(ctx, scene, camera28, params, host_out);
+  if (ctx && ctx->group) return lt_multi_render(ctx, scene, camera28, params, host_out, nullptr);
   LtLaunch L;
   int rc = check_params(ctx, scene, camera28, params, &L);
   if (rc != LT_OK) return rc;
@@ -1083,14 +1086,120 @@ extern "C" int lt_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, con
 
 extern "C" int lt_plugin_load(lt_ctx* ctx, const char* kernel_file_path, int* out_plugin_id) {
   if (!ctx || !kernel_file_path || !out_plugin_id) return fail(ctx, LT_ERR_INVALID, "lt_plugin_load: NULL argument");
-  if (ctx->group) return fail(ctx, LT_ERR_UNSUPPORTED, "lt_plugin_load: plug-in kernels run on single-GPU contexts");
+  std::string err;
+  LtPluginImage img;
+  if (!lt_plugin_compile(kernel_file_path, &img, &err)) return fail(ctx, LT_ERR_UNSUPPORTED, "lt_plugin_load: " + err);
+  if (ctx->group) return lt_multi_plugin_load(ctx, img, out_plugin_id);
   CK(cudaSetDevice(ctx->device));
   CK(cudaFree(0));  // make sure the primary context is current for the driver-API module load
-  std::string err;
-  LtPlugin* p = lt_plugin_compile(kernel_file_path, &err);
+  LtPlugin* p = lt_plugin_module_load(img, &err);
   if (!p) return fail(ctx, LT_ERR_UNSUPPORTED, "lt_plugin_load: " + err);
   ctx->plugins.push_back(p);
   *out_plugin_id = (int)ctx->plugins.size() - 1;
+  return LT_OK;
+}
+
+int lt_internal_render_plugin(lt_ctx* ctx, lt_scene* scene, const RefCamera& cam, const lt_render_params& P,
+                              const LtPluginRun& run, bool sync, const char* who) {
+  CK(cudaSetDevice(ctx->device));
+  LtPlugin* plugin = ctx->plugins[run.id];
+  const bool cl = lt_plugin_is_opencl_c(plugin);
+  const size_t floats = (size_t)P.width * P.height * P.depth;
+  int rc = ensure_out(ctx, floats);
+  if (rc != LT_OK) return rc;
+  // LT_ACCUM_NONE: every frame into the output, in order (F consecutive single-frame calls); otherwise every frame into
+  // the sample buffer, folded into the accumulator after it
+  const bool fold = P.accum_mode != LT_ACCUM_NONE;
+  if (fold && ctx->sampleFloats < floats) {
+    if (ctx->dSample) cudaFree(ctx->dSample);
+    ctx->dSample = nullptr;
+    ctx->sampleFloats = 0;
+    CK(cudaMalloc(&ctx->dSample, floats * sizeof(float)));
+    ctx->sampleFloats = floats;
+  }
+  float* dFrame = fold ? ctx->dSample : ctx->dOut;
+  if (ctx->cameraCount < P.frames) {
+    if (ctx->dCamera) cudaFree(ctx->dCamera);
+    ctx->dCamera = nullptr;
+    ctx->cameraCount = 0;
+    CK(cudaMalloc(&ctx->dCamera, sizeof(RefCamera) * (size_t)P.frames));
+    ctx->cameraCount = P.frames;
+  }
+  // frame k reads its own record, frameCount = camera.frameCount + k * frame_stride
+  const uint32_t stride = P.frame_stride ? P.frame_stride : 1u;
+  std::vector<RefCamera> cams((size_t)P.frames, cam);
+  for (int k = 0; k < P.frames; k++) cams[k].frameCount = cam.frameCount + (uint32_t)k * stride;
+  CK(cudaMemcpyAsync(ctx->dCamera, cams.data(), sizeof(RefCamera) * cams.size(), cudaMemcpyHostToDevice, ctx->stream));
+  std::string err;
+  if (!cl && lt_plugin_publish_scene(plugin, &scene->dev, ctx->stream, &err) != 0)
+    return fail(ctx, LT_ERR_CUDA, std::string(who) + ": " + err);
+  // pixels outside every work block (the remainder of W / wbx and H / wby) read 0; the reference leaves them undefined
+  if (cl) CK(cudaMemsetAsync(dFrame, 0, floats * sizeof(float), ctx->stream));
+  LtLaunch L = {};
+  L.width = P.width;
+  L.height = P.height;
+  L.depth = P.depth;
+  L.accumMode = P.accum_mode;
+  L.accumWeight = P.accum_weight;
+  CK(cudaEventRecord(ctx->ev0, ctx->stream));
+  int launches = 0;
+  for (int k = 0; k < P.frames; k++) {
+    const RefCamera* dCam = ctx->dCamera + k;
+    const int n = cl ? lt_plugin_launch_cl(plugin, run.kernelMode, scene->dNodes, scene->dPrims, scene->dMats,
+                                           scene->dLights, dCam, dFrame, P.width, P.height, P.depth, run.wbx, run.wby,
+                                           run.bx, run.by, ctx->stream, &err)
+                     : (lt_plugin_launch(plugin, run.kernelMode, &scene->dev, scene->dNodes, scene->dPrims, scene->dMats,
+                                         scene->dLights, dCam, dFrame, P.width, P.height, P.depth, run.bx, run.by,
+                                         ctx->stream, &err) == 0 ? 1 : -1);
+    if (n < 0) return fail(ctx, LT_ERR_CUDA, std::string(who) + ": " + err);
+    launches += n;
+    if (fold) {
+      L.cam = cams[k];
+      launches += lt_launch_plugin_accumulate(L, dFrame, ctx->dOut, ctx->stats.sm_count, ctx->stream);
+    }
+  }
+  CK(cudaGetLastError());
+  CK(cudaEventRecord(ctx->ev1, ctx->stream));
+  ctx->stats.kernel_launches = launches;
+  ctx->stats.rays = ctx->stats.node_tests = ctx->stats.tri_tests = 0;
+  ctx->stats.trace_ms = ctx->stats.shade_ms = ctx->stats.primary_shade_ms = ctx->stats.accumulate_ms = 0.0f;
+  ctx->stats.trace_launches = ctx->stats.shade_launches = 0;
+  if (sync) {
+    CK(cudaStreamSynchronize(ctx->stream));
+    CK(cudaEventElapsedTime(&ctx->stats.kernel_ms, ctx->ev0, ctx->ev1));
+  }
+  return LT_OK;
+}
+
+// Checks a plug-in id (and, for `cl` >= 0, its language) against the plug-ins of ctx; LT_ERR_INVALID otherwise.
+static int check_plugin(lt_ctx* ctx, int plugin_id, int cl, const char* who) {
+  const std::vector<LtPlugin*>& plugins = ctx->group ? lt_multi_plugins(ctx) : ctx->plugins;
+  if (plugin_id < 0 || plugin_id >= (int)plugins.size())
+    return fail(ctx, LT_ERR_INVALID, std::string(who) + ": bad argument");
+  if (cl == 0 && lt_plugin_is_opencl_c(plugins[plugin_id]))
+    return fail(ctx, LT_ERR_INVALID, std::string(who) + ": plug-in " + std::to_string(plugin_id) +
+                                         " is an OpenCL C kernel; launch it with lt_render_plugin_cl");
+  if (cl == 1 && !lt_plugin_is_opencl_c(plugins[plugin_id]))
+    return fail(ctx, LT_ERR_INVALID, std::string(who) + ": plug-in " + std::to_string(plugin_id) +
+                                         " is a CUDA kernel; launch it with lt_render_plugin");
+  return LT_OK;
+}
+
+// One frame, no accumulation, into ctx->dOut, then to host_out: the two single-frame entry points
+static int render_plugin_once(lt_ctx* ctx, lt_scene* scene, const void* camera28, const LtPluginRun& run, int width,
+                              int height, int depth, float* host_out, const char* who) {
+  lt_render_params P;
+  memset(&P, 0, sizeof P);
+  P.struct_size = sizeof P;
+  P.width = width;
+  P.height = height;
+  P.depth = depth;
+  P.frames = 1;
+  RefCamera cam;
+  memcpy(&cam, camera28, sizeof cam);
+  int rc = lt_internal_render_plugin(ctx, scene, cam, P, run, true, who);
+  if (rc != LT_OK) return rc;
+  if (host_out) return download(ctx, host_out, ctx->dOut, (size_t)width * height * depth * sizeof(float));
   return LT_OK;
 }
 
@@ -1098,30 +1207,11 @@ extern "C" int lt_render_plugin(lt_ctx* ctx, lt_scene* scene, const void* camera
                                 int width, int height, int depth, int block_x, int block_y, float* host_out) {
   if (!ctx) return fail(nullptr, LT_ERR_INVALID, "lt_render_plugin: ctx is NULL");
   if (ctx->group) return fail(ctx, LT_ERR_UNSUPPORTED, "lt_render_plugin: plug-in kernels run on single-GPU contexts");
-  if (!scene || !camera28 || plugin_id < 0 || plugin_id >= (int)ctx->plugins.size() || width <= 0 || height <= 0 ||
-      depth < 1)
+  if (!scene || !camera28 || width <= 0 || height <= 0 || depth < 1)
     return fail(ctx, LT_ERR_INVALID, "lt_render_plugin: bad argument");
-  if (lt_plugin_is_opencl_c(ctx->plugins[plugin_id]))
-    return fail(ctx, LT_ERR_INVALID, "lt_render_plugin: plug-in " + std::to_string(plugin_id) +
-                                         " is an OpenCL C kernel; launch it with lt_render_plugin_cl");
-  CK(cudaSetDevice(ctx->device));
-  size_t floats = (size_t)width * height * depth;
-  int rc = ensure_out(ctx, floats);
-  if (rc != LT_OK) return rc;
-  if (!ctx->dCamera) CK(cudaMalloc(&ctx->dCamera, sizeof(RefCamera)));
-  CK(cudaMemcpyAsync(ctx->dCamera, camera28, sizeof(RefCamera), cudaMemcpyHostToDevice, ctx->stream));
-  CK(cudaEventRecord(ctx->ev0, ctx->stream));
-  std::string err;
-  if (lt_plugin_launch(ctx->plugins[plugin_id], kernel_mode ? 1 : 0, &scene->dev, scene->dNodes, scene->dPrims, scene->dMats,
-                       scene->dLights, ctx->dCamera, ctx->dOut, width, height, depth, block_x, block_y, ctx->stream,
-                       &err) != 0)
-    return fail(ctx, LT_ERR_CUDA, "lt_render_plugin: " + err);
-  CK(cudaEventRecord(ctx->ev1, ctx->stream));
-  CK(cudaStreamSynchronize(ctx->stream));
-  CK(cudaEventElapsedTime(&ctx->stats.kernel_ms, ctx->ev0, ctx->ev1));
-  ctx->stats.kernel_launches = 1;
-  if (host_out) return download(ctx, host_out, ctx->dOut, floats * sizeof(float));
-  return LT_OK;
+  if (int rc = check_plugin(ctx, plugin_id, 0, "lt_render_plugin")) return rc;
+  const LtPluginRun run = {plugin_id, kernel_mode ? 1 : 0, block_x, block_y, 0, 0};
+  return render_plugin_once(ctx, scene, camera28, run, width, height, depth, host_out, "lt_render_plugin");
 }
 
 extern "C" int lt_render_plugin_cl(lt_ctx* ctx, lt_scene* scene, const void* camera28, int plugin_id, int kernel_mode,
@@ -1129,34 +1219,50 @@ extern "C" int lt_render_plugin_cl(lt_ctx* ctx, lt_scene* scene, const void* cam
                                    int group_y, float* host_out) {
   if (!ctx) return fail(nullptr, LT_ERR_INVALID, "lt_render_plugin_cl: ctx is NULL");
   if (ctx->group) return fail(ctx, LT_ERR_UNSUPPORTED, "lt_render_plugin_cl: plug-in kernels run on single-GPU contexts");
-  if (!scene || !camera28 || plugin_id < 0 || plugin_id >= (int)ctx->plugins.size() || width <= 0 || height <= 0 ||
-      depth < 1)
+  if (!scene || !camera28 || width <= 0 || height <= 0 || depth < 1)
     return fail(ctx, LT_ERR_INVALID, "lt_render_plugin_cl: bad argument");
-  if (!lt_plugin_is_opencl_c(ctx->plugins[plugin_id]))
-    return fail(ctx, LT_ERR_INVALID, "lt_render_plugin_cl: plug-in " + std::to_string(plugin_id) +
-                                         " is a CUDA kernel; launch it with lt_render_plugin");
+  if (int rc = check_plugin(ctx, plugin_id, 1, "lt_render_plugin_cl")) return rc;
   std::string err;
-  int wbx = work_block_x, wby = work_block_y, gx = group_x, gy = group_y;
-  if (!lt_plugin_cl_shape(width, height, &wbx, &wby, &gx, &gy, &err))
+  LtPluginRun run = {plugin_id, kernel_mode ? 1 : 0, group_x, group_y, work_block_x, work_block_y};
+  if (!lt_plugin_cl_shape(width, height, &run.wbx, &run.wby, &run.bx, &run.by, &err))
     return fail(ctx, LT_ERR_INVALID, "lt_render_plugin_cl: " + err);
-  CK(cudaSetDevice(ctx->device));
-  size_t floats = (size_t)width * height * depth;
-  int rc = ensure_out(ctx, floats);
+  return render_plugin_once(ctx, scene, camera28, run, width, height, depth, host_out, "lt_render_plugin_cl");
+}
+
+extern "C" int lt_render_plugin_frames(lt_ctx* ctx, lt_scene* scene, const void* camera28, int plugin_id,
+                                       const lt_render_params* params, int work_block_x, int work_block_y,
+                                       float* host_out) {
+  const char* who = "lt_render_plugin_frames";
+  if (!ctx) return fail(nullptr, LT_ERR_INVALID, "lt_render_plugin_frames: ctx is NULL");
+  if (!scene || !camera28 || !params) return fail(ctx, LT_ERR_INVALID, "lt_render_plugin_frames: NULL argument");
+  // lt_render's checks; kernel and max_ray_depth do not apply (a plug-in is its own kernel, with its own bounce cap)
+  lt_render_params P;
+  memset(&P, 0, sizeof P);
+  memcpy(&P, params, params->struct_size < sizeof P ? params->struct_size : sizeof P);
+  P.kernel = 0;
+  P.max_ray_depth = 0;
+  LtLaunch L;
+  if (int rc = launch_from_params(ctx, &P, &L, who)) return rc;
+  P.struct_size = sizeof P;
+  if (int rc = check_plugin(ctx, plugin_id, -1, who)) return rc;
+  if (P.flags & (LT_FLAG_STATS | LT_FLAG_STATS_TRACED | LT_FLAG_CULL))
+    return fail(ctx, LT_ERR_UNSUPPORTED, "lt_render_plugin_frames: a plug-in has no counters (LT_FLAG_STATS) and no "
+                                         "culled traversal (LT_FLAG_CULL)");
+  const bool cl = lt_plugin_is_opencl_c((ctx->group ? lt_multi_plugins(ctx) : ctx->plugins)[plugin_id]);
+  LtPluginRun run = {plugin_id, P.kernel_mode ? 1 : 0, P.block_x, P.block_y, work_block_x, work_block_y};
+  if (cl) {
+    std::string err;
+    if (!lt_plugin_cl_shape(P.width, P.height, &run.wbx, &run.wby, &run.bx, &run.by, &err))
+      return fail(ctx, LT_ERR_INVALID, "lt_render_plugin_frames: " + err);
+  } else if (work_block_x || work_block_y) {
+    return fail(ctx, LT_ERR_INVALID, "lt_render_plugin_frames: a work block applies to OpenCL C plug-ins only");
+  }
+  if (ctx->group) return lt_multi_render(ctx, scene, camera28, &P, host_out, &run);
+  RefCamera cam;
+  memcpy(&cam, camera28, sizeof cam);
+  int rc = lt_internal_render_plugin(ctx, scene, cam, P, run, true, who);
   if (rc != LT_OK) return rc;
-  if (!ctx->dCamera) CK(cudaMalloc(&ctx->dCamera, sizeof(RefCamera)));
-  CK(cudaMemcpyAsync(ctx->dCamera, camera28, sizeof(RefCamera), cudaMemcpyHostToDevice, ctx->stream));
-  // pixels outside every work block (the remainder of W / wbx and H / wby) read 0; the reference leaves them undefined
-  CK(cudaMemsetAsync(ctx->dOut, 0, floats * sizeof(float), ctx->stream));
-  CK(cudaEventRecord(ctx->ev0, ctx->stream));
-  int launches = lt_plugin_launch_cl(ctx->plugins[plugin_id], kernel_mode ? 1 : 0, scene->dNodes, scene->dPrims,
-                                     scene->dMats, scene->dLights, ctx->dCamera, ctx->dOut, width, height, depth, wbx, wby,
-                                     gx, gy, ctx->stream, &err);
-  if (launches < 0) return fail(ctx, LT_ERR_CUDA, "lt_render_plugin_cl: " + err);
-  CK(cudaEventRecord(ctx->ev1, ctx->stream));
-  CK(cudaStreamSynchronize(ctx->stream));
-  CK(cudaEventElapsedTime(&ctx->stats.kernel_ms, ctx->ev0, ctx->ev1));
-  ctx->stats.kernel_launches = launches;
-  if (host_out) return download(ctx, host_out, ctx->dOut, floats * sizeof(float));
+  if (host_out) return download(ctx, host_out, ctx->dOut, (size_t)P.width * P.height * P.depth * sizeof(float));
   return LT_OK;
 }
 

@@ -86,8 +86,16 @@ int lt_launch_render_wavefront(const LtSceneDev& sc, const LtPlan& plan, const L
 #include <utility>
 #include <vector>
 struct LtPlugin;
-LtPlugin* lt_plugin_compile(const char* path, std::string* err);
+// A compiled plug-in, not yet loaded on a device: compiled once, loaded on every device of a multi-GPU context.
+struct LtPluginImage {
+  std::string path;
+  bool openclC = false;
+  std::vector<char> cubin;
+};
+bool lt_plugin_compile(const char* path, LtPluginImage* img, std::string* err);
+LtPlugin* lt_plugin_module_load(const LtPluginImage& img, std::string* err);  // into the calling thread's current context
 void lt_plugin_free(LtPlugin* p);
+int lt_plugin_publish_scene(LtPlugin* p, const LtSceneDev* sceneDev, cudaStream_t stream, std::string* err);
 int lt_plugin_launch(LtPlugin* p, int kernelMode, const LtSceneDev* sceneDev, const void* dNodes, const void* dPrims,
                      const void* dMats, const void* dLights, const void* dCamera, float* dOut, int width, int height,
                      int depth, int bx, int by, cudaStream_t stream, std::string* err);
@@ -100,6 +108,16 @@ bool lt_plugin_cl_shape(int width, int height, int* wbx, int* wby, int* gx, int*
 int lt_plugin_launch_cl(LtPlugin* p, int kernelMode, const void* dNodes, const void* dPrims, const void* dMats,
                         const void* dLights, const void* dCamera, float* dOut, int width, int height, int depth, int wbx,
                         int wby, int gx, int gy, cudaStream_t stream, std::string* err);
+// k_plugin_accumulate (lt_kernels.cu): folds one plug-in frame (`sample`) into the accumulator `acc` with FrameSink, as
+// L.accumMode / L.accumWeight / L.cam.frameCount say; 3 channels per pixel at stride L.depth
+int lt_launch_plugin_accumulate(const LtLaunch& L, const float* sample, float* acc, int smCount, cudaStream_t stream);
+// What a plug-in call launches besides its frames (host-side only).
+struct LtPluginRun {
+  int id;
+  int kernelMode;
+  int bx, by;    // CUDA block of a .cu plug-in, work-group of a .cl plug-in
+  int wbx, wby;  // work block of a .cl plug-in (as normalised by lt_plugin_cl_shape)
+};
 
 // ---- context and scene objects behind the C-ABI handles (lt_capi.cu; lt_multi.cu for multi-GPU contexts) ----
 #include <vector>
@@ -121,7 +139,10 @@ struct lt_ctx {
   std::vector<cudaEvent_t> traceEvents;  // pairs of events around launches (timed when synchronous)
   std::vector<unsigned char> pairKinds;  // LT_TIMED_* of every pair
   std::vector<LtPlugin*> plugins;  // compiled user kernels, by id
-  RefCamera* dCamera = nullptr;    // camera buffer for plug-in launches
+  RefCamera* dCamera = nullptr;    // camera records of a plug-in call, one per frame
+  int cameraCount = 0;
+  float* dSample = nullptr;        // one plug-in frame of an accumulating call, folded into dOut
+  size_t sampleFloats = 0;
   void* wfWorkspace = nullptr;  // wavefront path state / ray queues (two batch workspaces when batches overlap)
   size_t wfBytes = 0;
   LtWfAux wfAux = {};           // second stream + events for overlapping consecutive wavefront batches
@@ -154,7 +175,11 @@ int lt_multi_scene_upload(lt_ctx* ctx, const void* nodes, uint64_t node_bytes, c
                           uint64_t primitive_bytes, const void* materials, uint64_t material_bytes,
                           const void* light_container, uint64_t light_bytes, lt_scene** out_scene);
 void lt_multi_scene_release(lt_ctx* ctx, lt_scene* scene);
-int lt_multi_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params, float* host_out);
+// run: NULL renders the built-in kernel of params, otherwise the plug-in of run (loaded on every device)
+int lt_multi_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params, float* host_out,
+                    const LtPluginRun* run);
+int lt_multi_plugin_load(lt_ctx* ctx, const LtPluginImage& img, int* out_plugin_id);
+const std::vector<LtPlugin*>& lt_multi_plugins(const lt_ctx* ctx);  // device 0's; every device holds the same ids
 void lt_multi_destroy(lt_ctx* ctx);
 int lt_multi_accum_reset(lt_ctx* ctx);
 int lt_internal_fail(lt_ctx* ctx, int code, const std::string& msg);  // sets the context's (and the thread's) last error
@@ -164,6 +189,10 @@ int lt_internal_download(lt_ctx* ctx, float* host_out, const float* dSrc, size_t
 // one device's share of a render call: like lt_render_device, with the row window of a tile split
 int lt_internal_render_rows(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params,
                             float* device_out, int fullHeight, int rowBlock, int rowStride, int rowPhase, int sync);
+// params->frames frames of a plug-in into ctx->dOut, combined by params->accum_mode (arguments already checked); `who`
+// names the entry point in error messages
+int lt_internal_render_plugin(lt_ctx* ctx, lt_scene* scene, const RefCamera& cam, const lt_render_params& P,
+                              const LtPluginRun& run, bool sync, const char* who);
 
 // device-side BVH construction in the reference's flattened layout (lt_bvh.cu)
 enum LtBvhBuilder { LT_BVH_LBVH, LT_BVH_PLOC };

@@ -381,6 +381,22 @@ __global__ void k_build_tris(const RefPrim* __restrict__ prims, int n, LtTri* __
   tris[i] = t;
 }
 
+// One frame of a plug-in (lt_render_plugin_frames) folded into the accumulator: the arithmetic of the built-in
+// pipelines' FrameSink for the frame with frameCount L.cam.frameCount, one pixel per thread.  Per pixel at depth 3 it
+// reads 12 B of sample and 12 B of accumulator and writes 12 B.
+__global__ void k_plugin_accumulate(LtLaunch L, const float* __restrict__ sample, float* __restrict__ acc,
+                                    long long pixels) {
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < pixels; i += stride) {
+    const long long id = i * L.depth;
+    const float c[3] = {sample[id + 0], sample[id + 1], sample[id + 2]};
+    FrameSink sink;
+    sink.begin(L, acc, id);
+    sink.frame(L, L.cam.frameCount, c);
+    sink.end(acc, id);
+  }
+}
+
 // ------------------------------------------------------------------------------------------------
 // host-side launchers
 // ------------------------------------------------------------------------------------------------
@@ -392,6 +408,13 @@ int lt_launch_debug_random(const float* fx, const float* fy, const float* seed, 
 int lt_launch_debug_hemisphere(const float* u1, const float* u2, const float* up, int n, float* out,
                                cudaStream_t stream) {
   k_debug_hemisphere<<<(n + 255) / 256, 256, 0, stream>>>(u1, u2, up, n, out);
+  return 1;
+}
+
+int lt_launch_plugin_accumulate(const LtLaunch& L, const float* sample, float* acc, int smCount, cudaStream_t stream) {
+  const long long pixels = (long long)L.width * L.height;
+  const long long need = (pixels + 255) / 256, cap = (long long)smCount * 8;
+  k_plugin_accumulate<<<(unsigned)(need < cap ? need : cap), 256, 0, stream>>>(L, sample, acc, pixels);
   return 1;
 }
 

@@ -216,6 +216,35 @@ int lt_multi_accum_reset(lt_ctx* ctx) {
   return LT_OK;
 }
 
+// One compiled image, loaded on every device in that device's thread (its primary context current there): each
+// device's context holds the plug-in under the same id.
+int lt_multi_plugin_load(lt_ctx* ctx, const LtPluginImage& img, int* out_plugin_id) {
+  LtGroup* g = ctx->group;
+  const size_t G = g->ctx.size();
+  std::vector<LtPlugin*> loaded(G, nullptr);
+  std::vector<std::string> errs(G);
+  std::vector<std::thread> workers;
+  for (size_t k = 0; k < G; k++)
+    workers.emplace_back([&, k]() {
+      if (cudaSetDevice(g->ctx[k]->device) != cudaSuccess || cudaFree(0) != cudaSuccess) {
+        errs[k] = "cannot make device " + std::to_string(g->ctx[k]->device) + " current";
+        return;
+      }
+      loaded[k] = lt_plugin_module_load(img, &errs[k]);
+    });
+  for (std::thread& t : workers) t.join();
+  for (size_t k = 0; k < G; k++)
+    if (!loaded[k]) {
+      for (LtPlugin* p : loaded) lt_plugin_free(p);
+      return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED, "lt_plugin_load: " + errs[k]);
+    }
+  for (size_t k = 0; k < G; k++) g->ctx[k]->plugins.push_back(loaded[k]);
+  *out_plugin_id = (int)g->ctx[0]->plugins.size() - 1;
+  return LT_OK;
+}
+
+const std::vector<LtPlugin*>& lt_multi_plugins(const lt_ctx* ctx) { return ctx->group->ctx[0]->plugins; }
+
 static bool ensure_nccl(LtGroup* g, std::string* why) {
   if (g->ncclTried) return g->ncclReady;
   g->ncclTried = true;
@@ -308,28 +337,34 @@ extern "C" int lt_debug_tile_rows(int height, int devices, int device, int32_t* 
   return rows;
 }
 
-int lt_multi_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params, float* host_out) {
+int lt_multi_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params, float* host_out,
+                    const LtPluginRun* run) {
   LtGroup* g = ctx->group;
-  if (!scene || !camera28 || !params) return lt_internal_fail(ctx, LT_ERR_INVALID, "lt_render: NULL argument");
+  const std::string who = run ? "lt_render_plugin_frames: " : "lt_render: ";
+  if (!scene || !camera28 || !params) return lt_internal_fail(ctx, LT_ERR_INVALID, who + "NULL argument");
   if (scene->parts.size() != g->ctx.size())
-    return lt_internal_fail(ctx, LT_ERR_INVALID, "lt_render: the scene was not uploaded through this multi-GPU context");
+    return lt_internal_fail(ctx, LT_ERR_INVALID, who + "the scene was not uploaded through this multi-GPU context");
   if (params->struct_size != sizeof(lt_render_params) && params->struct_size != offsetof(lt_render_params, split_mode))
-    return lt_internal_fail(ctx, LT_ERR_INVALID, "lt_render: params.struct_size mismatch");
+    return lt_internal_fail(ctx, LT_ERR_INVALID, who + "params.struct_size mismatch");
   lt_render_params P;
   memset(&P, 0, sizeof P);
   memcpy(&P, params, params->struct_size < sizeof P ? params->struct_size : sizeof P);
   P.struct_size = sizeof P;
   if (P.width <= 0 || P.height <= 0 || P.depth < 3 || P.frames < 1)
-    return lt_internal_fail(ctx, LT_ERR_INVALID, "lt_render: width/height must be > 0, depth >= 3, frames >= 1");
+    return lt_internal_fail(ctx, LT_ERR_INVALID, who + "width/height must be > 0, depth >= 3, frames >= 1");
   if (P.flags & LT_FLAG_STATS)
-    return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED, "lt_render: LT_FLAG_STATS counts on a single-GPU context");
+    return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED, who + "LT_FLAG_STATS counts on a single-GPU context");
   const int G = (int)g->ctx.size();
   int split = P.split_mode;
-  if (split == LT_SPLIT_AUTO) split = (P.frames >= 2 && P.accum_mode != LT_ACCUM_NONE) ? LT_SPLIT_SAMPLES : LT_SPLIT_TILES;
+  // a plug-in derives its pixel from blockIdx / get_global_id: it cannot be given a subset of the rows
+  if (run && split == LT_SPLIT_TILES)
+    return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED, who + "a plug-in cannot render a tile split (use LT_SPLIT_SAMPLES)");
+  if (split == LT_SPLIT_AUTO)
+    split = (run || (P.frames >= 2 && P.accum_mode != LT_ACCUM_NONE)) ? LT_SPLIT_SAMPLES : LT_SPLIT_TILES;
   if (split == LT_SPLIT_SAMPLES && P.accum_mode == LT_ACCUM_NONE)
     return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED,
-                            "lt_render: a sample split needs an accumulating call (LT_ACCUM_NONE keeps only the last frame)");
-  if (split != LT_SPLIT_SAMPLES && split != LT_SPLIT_TILES) return lt_internal_fail(ctx, LT_ERR_INVALID, "lt_render: bad split_mode");
+                            who + "a sample split needs an accumulating call (LT_ACCUM_NONE keeps only the last frame)");
+  if (split != LT_SPLIT_SAMPLES && split != LT_SPLIT_TILES) return lt_internal_fail(ctx, LT_ERR_INVALID, who + "bad split_mode");
   RefCamera cam;
   memcpy(&cam, camera28, sizeof cam);
   const size_t fullFloats = (size_t)P.width * P.height * P.depth;
@@ -383,7 +418,7 @@ int lt_multi_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt
   } else {
     // ---- sample split ----
     if (P.accum_mode == LT_ACCUM_RUNNING_MEAN && stride != 1u)
-      return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED, "lt_render: a multi-GPU running mean needs frame_stride 1");
+      return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED, who + "a multi-GPU running mean needs frame_stride 1");
     const bool mean = P.accum_mode == LT_ACCUM_RUNNING_MEAN;
     // running mean: new = old * fc/(fc+F) + sum(samples)/(fc+F)  (fc = frames already in the accumulator; 0 discards it,
     // like frameCount == 0 in accumulator.frag:10-19)
@@ -394,7 +429,7 @@ int lt_multi_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt
     const char* ex = getenv("LT_MULTI_EXCHANGE");
     bool useNccl = !(ex && strcmp(ex, "p2p") == 0) && ensure_nccl(g, &why);
     if (!useNccl && !ensure_peers(g, fullFloats, &why))
-      return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED, "lt_render: no way to combine the devices' accumulators: " + why);
+      return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED, who + "no way to combine the devices' accumulators: " + why);
     for (int k = 0; k < G; k++)
       workers.emplace_back([&, k]() {
         lt_ctx* c = g->ctx[k];
@@ -418,7 +453,8 @@ int lt_multi_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt
           Pk.split_mode = 0;
           RefCamera ck = cam;
           ck.frameCount = cam.frameCount + (uint32_t)k * stride;
-          rcs[k] = lt_internal_render_rows(c, scene->parts[k], &ck, &Pk, c->dOut, P.height, P.height, 1, 0, 0);
+          rcs[k] = run ? lt_internal_render_plugin(c, scene->parts[k], ck, Pk, *run, false, "lt_render_plugin_frames")
+                       : lt_internal_render_rows(c, scene->parts[k], &ck, &Pk, c->dOut, P.height, P.height, 1, 0, 0);
         }
         cudaEventRecord(g->rendered[k], c->stream);
       });

@@ -5,8 +5,8 @@
 //   (LinearBVHNode*, Primitive*, Material*, LightContainer*, Camera*, float* out, int W, int H, int depth)
 // (src/cuda/renderer_cuda.cpp:20-39,67-72,113-133; resources/kernels/cuda/basic.cu:331-340).  The seven
 // shipped kernels map to built-in pipelines; any OTHER .cu file goes through here: compiled once per
-// context for sm_100a, cached, and launched on the buffers of the uploaded scene in the reference's
-// layouts.  NVRTC and the driver API are loaded lazily with dlopen so that liblt_b200.so itself has no
+// context for sm_100a (once for all devices of a multi-GPU context, which loads the cubin on each), cached, and
+// launched on the buffers of the uploaded scene in the reference's layouts.  NVRTC and the driver API are loaded lazily with dlopen so that liblt_b200.so itself has no
 // link-time dependency on them (it must load on machines without a GPU).
 #include <cuda.h>
 #include <dlfcn.h>
@@ -406,38 +406,43 @@ bool lt_plugin_compile_cl_only(const char* path, std::string* err) {
   return true;
 }
 
-// Compiles `path` (a .cl file as OpenCL C, anything else as CUDA); on failure returns nullptr and the compiler log /
-// reason in `err`.
-LtPlugin* lt_plugin_compile(const char* path, std::string* err) {
+// Compiles `path` (a .cl file as OpenCL C, anything else as CUDA) to an sm_100a cubin; on failure returns false and
+// the compiler log / reason in `err`.  No device is touched: a multi-GPU context loads the one image on every device.
+bool lt_plugin_compile(const char* path, LtPluginImage* img, std::string* err) {
   if (!load_api()) {
     *err = "plug-in kernels need NVRTC and the CUDA driver: " + g_api.why;
-    return nullptr;
+    return false;
   }
   const bool openclC = has_suffix(path, ".cl");
   std::string program;
   bool contractOff = false;
   std::vector<std::string> entries;
-  if (openclC ? !cl_source(path, &program, &contractOff, &entries, err) : !read_text(path, &program, err)) return nullptr;
-  std::vector<char> cubin;
-  if (!nvrtc_cubin(program, path, openclC, contractOff, &cubin, err)) return nullptr;
+  if (openclC ? !cl_source(path, &program, &contractOff, &entries, err) : !read_text(path, &program, err)) return false;
+  img->path = path;
+  img->openclC = openclC;
+  return nvrtc_cubin(program, path, openclC, contractOff, &img->cubin, err);
+}
+
+// Loads a compiled image into the context current on the calling thread; nullptr with the reason in `err` on failure.
+LtPlugin* lt_plugin_module_load(const LtPluginImage& img, std::string* err) {
   LtPlugin* p = new LtPlugin();
-  p->path = path;
-  p->openclC = openclC;
-  if (g_api.moduleLoadData(&p->module, cubin.data()) != CUDA_SUCCESS) {
+  p->path = img.path;
+  p->openclC = img.openclC;
+  if (g_api.moduleLoadData(&p->module, img.cubin.data()) != CUDA_SUCCESS) {
     *err = "cuModuleLoadData failed for the compiled plug-in";
     delete p;
     return nullptr;
   }
   g_api.moduleGetFunction(&p->linear, p->module, "linearKernel");
   g_api.moduleGetFunction(&p->tile, p->module, "tileKernel");
-  if (!openclC) {
+  if (!p->openclC) {
     size_t bytes = 0;
     CUdeviceptr addr = 0;
     if (g_api.moduleGetGlobal(&addr, &bytes, p->module, "lt_scene") == CUDA_SUCCESS && bytes == sizeof(LtSceneDev))
       p->sceneSymbol = addr;
   }
   if (!p->linear && !p->tile) {
-    *err = std::string(path) + " exports neither linearKernel nor tileKernel (extern \"C\" __global__)";
+    *err = p->path + " exports neither linearKernel nor tileKernel (extern \"C\" __global__)";
     g_api.moduleUnload(p->module);
     delete p;
     return nullptr;
@@ -453,17 +458,24 @@ void lt_plugin_free(LtPlugin* p) {
   delete p;
 }
 
-// Launch shape of the reference: grid = ceil(W/bx) x ceil(H/by), block = bx x by (32x1 for MAX_FIT,
-// src/cuda/renderer_cuda.cpp:74-88).  Returns 0, or -1 with `err` set.
-int lt_plugin_launch(LtPlugin* p, int kernelMode, const LtSceneDev* sceneDev, const void* dNodes, const void* dPrims,
-                     const void* dMats, const void* dLights, const void* dCamera, float* dOut, int width, int height,
-                     int depth, int bx, int by, cudaStream_t stream, std::string* err) {
-  CUfunction fn = kernelMode ? p->tile : p->linear;
+// Sets the plug-in's `lt_scene` (if it uses the device API) to the scene the following launches render.  Returns 0, or
+// -1 with `err` set.
+int lt_plugin_publish_scene(LtPlugin* p, const LtSceneDev* sceneDev, cudaStream_t stream, std::string* err) {
   if (p->sceneSymbol && sceneDev &&
       g_api.memcpyHtoDAsync(p->sceneSymbol, sceneDev, sizeof(LtSceneDev), (CUstream)stream) != CUDA_SUCCESS) {
     *err = "cannot set lt_scene of plug-in " + p->path;
     return -1;
   }
+  return 0;
+}
+
+// Launch shape of the reference: grid = ceil(W/bx) x ceil(H/by), block = bx x by (32x1 for MAX_FIT,
+// src/cuda/renderer_cuda.cpp:74-88).  sceneDev (published by lt_plugin_publish_scene) sizes the traversal stacks.
+// Returns 0, or -1 with `err` set.
+int lt_plugin_launch(LtPlugin* p, int kernelMode, const LtSceneDev* sceneDev, const void* dNodes, const void* dPrims,
+                     const void* dMats, const void* dLights, const void* dCamera, float* dOut, int width, int height,
+                     int depth, int bx, int by, cudaStream_t stream, std::string* err) {
+  CUfunction fn = kernelMode ? p->tile : p->linear;
   if (!fn) {
     *err = p->path + (kernelMode ? " has no tileKernel" : " has no linearKernel");
     return -1;

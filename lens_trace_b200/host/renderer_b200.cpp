@@ -151,9 +151,11 @@ void RendererB200::renderCommon(const std::string& kernelFilePath, KernelMode ke
     p = e->pNext;
   }
 
-  // which context renders: the multi-GPU one when the extension asks for several devices (built-in pipelines only)
-  const uint32_t wantDevices = (ext && ext->deviceCount > 1 && plugin < 0) ? ext->deviceCount : 1;
+  // which context renders: the multi-GPU one when the extension asks for several devices (a plug-in splits samples
+  // only, so it needs an accumulating call there)
+  const uint32_t wantDevices = (ext && ext->deviceCount > 1 && (plugin < 0 || ext->accumulate)) ? ext->deviceCount : 1;
   if (wantDevices > 1 && (groupCtx == nullptr || groupDevices != wantDevices)) {
+    groupPluginCache.clear();
     for (size_t i = 0; i < sceneCache.size(); i++)
       if (sceneCache[i].groupScene) {
         lt_scene_release(groupCtx, sceneCache[i].groupScene);
@@ -171,6 +173,22 @@ void RendererB200::renderCommon(const std::string& kernelFilePath, KernelMode ke
     groupDevices = wantDevices;
   }
   lt_ctx* useCtx = wantDevices > 1 ? groupCtx : ctx;
+  if (plugin >= 0 && wantDevices > 1) {  // the same file, loaded on the devices of the group
+    std::map<std::string, int>::iterator pc = groupPluginCache.find(kernelFilePath);
+    if (pc != groupPluginCache.end()) {
+      plugin = pc->second;
+    } else {
+      if (lt_plugin_load(groupCtx, Resource::findResource(kernelFilePath).c_str(), &plugin) != LT_OK) {
+        printf("%s\n", lt_last_error(groupCtx));
+        plugin = -1;
+      }
+      groupPluginCache[kernelFilePath] = plugin;
+    }
+    if (plugin < 0) {
+      printf("Kernel Error: '%s' could not be loaded on %u devices\n", kernelFilePath.c_str(), wantDevices);
+      return;
+    }
+  }
   CachedScene* entry = nullptr;
   for (size_t i = 0; i < sceneCache.size(); i++) {
     CachedScene& c = sceneCache[i];
@@ -226,7 +244,7 @@ void RendererB200::renderCommon(const std::string& kernelFilePath, KernelMode ke
     params.frames = ext->frames ? (int)ext->frames : 1;
     params.accum_mode = ext->accumulate ? LT_ACCUM_RUNNING_MEAN : LT_ACCUM_NONE;
     params.max_ray_depth = (int)ext->maxRayDepth;
-    if (ext->collectStats && wantDevices == 1) params.flags |= LT_FLAG_STATS;
+    if (ext->collectStats && wantDevices == 1 && plugin < 0) params.flags |= LT_FLAG_STATS;
     params.split_mode = (int)ext->splitMode;
   }
   uint64_t need = sizeof(float) * imageDimensions[0] * imageDimensions[1] * imageDimensions[2];
@@ -236,7 +254,12 @@ void RendererB200::renderCommon(const std::string& kernelFilePath, KernelMode ke
     return;
   }
   int rc;
-  if (plugin >= 0 && isCl)
+  if (plugin >= 0 && ext)  // frames, accumulation and devices as the extension asks
+    rc = lt_render_plugin_frames(useCtx, scene, camera->getCameraBuffer(), plugin, &params,
+                                 isCl && workBlockSize ? (int)workBlockSize[0] : 0,
+                                 isCl && workBlockSize ? (int)workBlockSize[1] : 0,
+                                 (float*)pOutputBuffer);
+  else if (plugin >= 0 && isCl)
     rc = lt_render_plugin_cl(ctx, scene, camera->getCameraBuffer(), plugin, params.kernel_mode, params.width,
                              params.height, params.depth, workBlockSize ? (int)workBlockSize[0] : 0,
                              workBlockSize ? (int)workBlockSize[1] : 0, params.block_x, params.block_y,
