@@ -227,10 +227,25 @@ int lt_debug_tile_rows(int height, int devices, int device, int32_t* out_rows, i
  * Exposed so that the layout can be checked against the reference traversal on a machine without a GPU. */
 int lt_debug_build_threaded(const void* nodes, uint64_t node_bytes, void* out_records);
 
-/* Host-only: the eight pruned copies lt_scene_upload builds beside those (same record format, inner nodes that
- * cannot change which leaves a ray reaches left out; skip links index out_records).  *out_stride receives the
- * records per copy; out_records (8 * stride * 32 bytes, at most 8 * node_count * 32) may be NULL to ask for it. */
+/* Host-only: the eight pruned copies of the reference tree (same record format, inner nodes that cannot change which
+ * leaves a ray reaches left out; skip links index out_records), which lt_scene_upload builds beside those when it
+ * builds no traversal tree.  *out_stride receives the records per copy; out_records (8 * stride * 32 bytes, at most
+ * 8 * node_count * 32) may be NULL to ask for it. */
 int lt_debug_build_threaded_pruned(const void* nodes, uint64_t node_bytes, void* out_records, int32_t* out_stride);
+
+/* Host-only: every threaded record lt_scene_upload builds for a small tree whose leaves link primitives below
+ * prim_count.  out_records (16 * node_count * 32 bytes of room): the eight full copies, then the eight pruned copies
+ * (*out_stride records each; skip links absolute, from record 8 * node_count).  When every leaf box lies inside all
+ * its ancestors' boxes (bounds finite, lo <= hi, no primitive linked twice, inner root), the pruned copies are those
+ * of a traversal tree: a SAH tree over the reference's leaves that reaches the same leaves in another order.  Then
+ * *out_traversal = 1 and out_rank (8 * prim_count int32) receives the tie-break table rank[o][p] (LtSceneDev::rank);
+ * otherwise *out_traversal = 0, the pruned copies are lt_debug_build_threaded_pruned's and out_rank is not written. */
+int lt_debug_build_traversal_tree(const void* nodes, uint64_t node_bytes, int32_t prim_count, void* out_records,
+                                  int32_t* out_stride, int32_t* out_rank, int32_t* out_traversal);
+
+/* Test hook: 1 when the pruned threaded copies of an uploaded scene are a traversal tree, 0 when not (also for
+ * scenes without host-built copies), < 0 on error. */
+int lt_debug_scene_traversal_tree(const lt_scene* scene);
 
 /* Test hook: full != 0 makes launches on `scene` (single-GPU) walk the full threaded copies for every ray, 0 restores
  * the pruned ones.  The output is the same either way; tests compare the two. */

@@ -89,8 +89,12 @@ static_assert(sizeof(LtTri) == 48, "triangle record is 48 bytes");
 // Host-built copies are followed by eight PRUNED copies (copy o at records prunedBase + o * prunedStride): the
 // same sequences without the inner nodes whose two child boxes lie inside their own box and which a ray that
 // entered the nearest kept ancestor usually enters too.  For a ray with finite, nonzero direction reciprocals and a
-// finite origin a contained child is hit only if its parent is, so the walk records the same leaves in the same
-// order; every other ray starts in the full copies.  One 32-byte sector, two 128-bit loads.
+// finite origin a contained child is hit only if its parent is, so the walk records the same leaves; every other ray
+// starts in the full copies.  When every leaf box lies inside all its ancestors' boxes, that argument makes a leaf's
+// reach depend on its own box alone, and the pruned copies are those of a TRAVERSAL TREE: a SAH tree over the
+// reference's leaves (each copied as is: box, primitive, count) with exact min/max inner boxes.  It reaches the same
+// leaves in another order; LtSceneDev::rank restores the reference's choice among hits of equal t.  Otherwise they
+// are pruned copies of the reference tree itself, in the reference's order.  One 32-byte sector, two 128-bit loads.
 struct __align__(16) LtThreadNode {
   float4 a;  // lo.x lo.y lo.z hi.x      lo = dirIsNeg ? boundsMax : boundsMin, hi the other one
   float4 b;  // hi.y hi.z bits(link) bits(skip)   link < 0: leaf, ~primitivesOffset; >= 0: inner node
@@ -115,6 +119,9 @@ struct LtSceneDev {
   int prunedBase, prunedStride;  // pruned copy o of tnodes: records [prunedBase + o * prunedStride, + prunedStride);
                                  // 0 and nodeCount: the full copies (tnodesCoherent, or no pruned copies)
   const LtThreadNode* tnodes;  // 8 * nodeCount full threaded records, then the pruned ones, or NULL (scene too large)
+  const int* rank;  // [8][primCount]: position, in octant o's reference visit order, of the leaf whose primitive is p;
+                    // set when the pruned copies are a traversal tree (NULL otherwise).  The reference keeps the first
+                    // of several triangles with equal t, i.e. the least (t, rank): tri_test breaks equal-t ties by it
   const LtThreadNode* tnodesCoherent;  // the same records for a large scene (built on the device), used only by the
                                        // lighting kernels' megakernel launches (camera rays + shadow rays towards a
                                        // light): incoherent rays spread over eight copies that no longer fit in L2

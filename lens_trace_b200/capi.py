@@ -19,7 +19,8 @@ SYMBOLS = [
     "lt_scene_release", "lt_render", "lt_render_device", "lt_accum_reset", "lt_accum_read", "lt_primary_hits",
     "lt_last_stats", "lt_kernel_from_path", "lt_kernel_name", "lt_debug_random", "lt_debug_hemisphere", "lt_debug_build_threaded", "lt_debug_build_threaded_pruned", "lt_debug_scene_full_threaded", "lt_plugin_load", "lt_render_plugin", "lt_render_plugin_cl", "lt_debug_compile_cl", "lt_debug_translate_cl", "lt_primary_hits_flags", "lt_scene_build_lbvh", "lt_scene_build_ploc", "lt_scene_download", "lt_scene_info",
     "lt_debug_gather_peak", "lt_ctx_create_multi", "lt_ctx_device_count", "lt_host_register", "lt_host_unregister", "lt_debug_tile_rows",
-    "lt_debug_plan", "lt_debug_ctx_limits", "lt_render_plugin_frames",
+    "lt_debug_plan", "lt_debug_ctx_limits", "lt_render_plugin_frames", "lt_debug_build_traversal_tree",
+    "lt_debug_scene_traversal_tree",
 ]
 
 
@@ -90,6 +91,9 @@ def load():
     lib.lt_debug_build_threaded.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p]
     lib.lt_debug_build_threaded_pruned.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.POINTER(C.c_int32)]
     lib.lt_debug_scene_full_threaded.argtypes = [C.c_void_p, C.c_int]
+    lib.lt_debug_build_traversal_tree.argtypes = [C.c_void_p, C.c_uint64, C.c_int32, C.c_void_p, C.POINTER(C.c_int32),
+                                                  C.c_void_p, C.POINTER(C.c_int32)]
+    lib.lt_debug_scene_traversal_tree.argtypes = [C.c_void_p]
     lib.lt_debug_ctx_limits.argtypes = [C.c_void_p, C.c_int, C.c_int]
     lib.lt_debug_plan.argtypes = [C.POINTER(RenderParams), C.c_uint64, C.c_int32, C.c_uint64, C.c_int32,
                                   C.POINTER(C.c_int64)]
@@ -315,6 +319,12 @@ class Context:
         with finite, nonzero reciprocals walk the pruned ones again (full=False, the default after upload)."""
         self._check(self.lib.lt_debug_scene_full_threaded(scene.h, 1 if full else 0), "lt_debug_scene_full_threaded")
 
+    def uses_traversal_tree(self, scene):
+        """Test hook: do the pruned threaded copies of `scene` walk a traversal tree (build_traversal_tree)?"""
+        rc = self.lib.lt_debug_scene_traversal_tree(scene.h)
+        self._check(min(rc, 0), "lt_debug_scene_traversal_tree")
+        return rc == 1
+
     def debug_limits(self, threaded_max_nodes, stream_min_nodes):
         """Test hook: trees of at most threaded_max_nodes nodes get host-built threaded copies at upload (larger ones
         device-built copies); deterministic launches on scenes of at least stream_min_nodes nodes run k_flat_stream."""
@@ -393,3 +403,25 @@ def build_threaded_pruned(nodes):
     if rc != 0:
         raise LtError("lt_debug_build_threaded_pruned failed (%d): %s" % (rc, lib.lt_last_error(None).decode()))
     return np.ascontiguousarray(out.reshape(-1)[:8 * stride.value].reshape(8, stride.value))
+
+
+def build_traversal_tree(nodes, prim_count):
+    """Host-only: the threaded records lt_scene_upload builds for a small tree (lt_debug_build_traversal_tree), as a
+    dict: "full" (8 x N, the reference's copies), "pruned" (8 x stride; skip links index it flattened, like
+    build_threaded_pruned), "stride", "traversal" (whether the pruned copies are a traversal tree over the reference's
+    leaves rather than the reference tree) and "rank" (8 x prim_count, the equal-t tie-break table, or None)."""
+    lib = load()
+    nodes = np.ascontiguousarray(nodes)
+    n = len(nodes)
+    out = np.zeros(16 * n, THREAD_NODE)
+    rank = np.zeros((8, prim_count), np.int32)
+    stride, trav = C.c_int32(0), C.c_int32(0)
+    rc = lib.lt_debug_build_traversal_tree(nodes.ctypes.data, nodes.nbytes, prim_count, out.ctypes.data,
+                                           C.byref(stride), rank.ctypes.data, C.byref(trav))
+    if rc != 0:
+        raise LtError("lt_debug_build_traversal_tree failed (%d): %s" % (rc, lib.lt_last_error(None).decode()))
+    k = stride.value
+    pruned = out[8 * n:8 * n + 8 * k].copy()
+    pruned["skip"] = np.where(pruned["skip"] == -2147483648, pruned["skip"], pruned["skip"] - 8 * n)
+    return {"full": out[:8 * n].reshape(8, n).copy(), "pruned": pruned.reshape(8, k), "stride": k,
+            "traversal": trav.value == 1, "rank": rank if trav.value == 1 else None}

@@ -9,6 +9,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <atomic>
 #include <cmath>
 #include <condition_variable>
@@ -390,6 +391,7 @@ extern "C" void lt_scene_release(lt_ctx* ctx, lt_scene* s) {
   cudaFree(s->dWide);
   cudaFree(s->dTris);
   cudaFree(s->dThread);
+  cudaFree(s->dRank);
   cudaFree(s->dThreadBig);
   delete s;
 }
@@ -397,6 +399,25 @@ extern "C" void lt_scene_release(lt_ctx* ctx, lt_scene* s) {
 // Threaded form of the tree (LtThreadNode, lens_trace_b200_device.cuh): eight copies of the node array, copy o in
 // the order the reference's traversal visits the nodes for rays of sign octant o, then eight pruned copies.  Built
 // on the host, for small trees only (lt_plan_threaded_copies).
+
+// The order in which the reference's traversal visits the nodes for rays of sign octant o (bit k: negative direction
+// on axis k), whole tree, no culling.
+static void visit_order(const RefNode* nodes, int o, std::vector<int>& order) {
+  std::vector<int> stack(1, 0);
+  order.clear();
+  while (!stack.empty()) {
+    int i = stack.back();
+    stack.pop_back();
+    order.push_back(i);
+    const RefNode& r = nodes[i];
+    if (r.primitiveCount == 0) {
+      bool neg = (o >> r.axis) & 1;  // basic.cu:180-186: second child first when the direction is negative
+      int nearC = neg ? r.offset : i + 1, farC = neg ? i + 1 : r.offset;
+      stack.push_back(farC);
+      stack.push_back(nearC);
+    }
+  }
+}
 
 // Appends eight copies of the threaded form to `out`, each in the visit order of its sign octant, leaving out the
 // nodes with keep[i] == 0.  Copy o is records [base + o * stride, base + (o + 1) * stride), base = out.size() on
@@ -408,26 +429,12 @@ static int append_threaded(const RefNode* nodes, int n, const std::vector<char>&
   int stride = 0;
   for (char k : keep) stride += k ? 1 : 0;
   out.resize((size_t)base + 8 * (size_t)stride);
-  std::vector<int> size(n), order, before(n + 1), stack;
+  std::vector<int> size(n), order, before(n + 1);
   for (int i = n - 1; i >= 0; i--)  // children follow their parent in the depth-first array
     size[i] = nodes[i].primitiveCount > 0 ? 1 : 1 + size[i + 1] + size[nodes[i].offset];
   auto bitsf = [](int v) { float f; memcpy(&f, &v, 4); return f; };
   for (int o = 0; o < 8; o++) {
-    order.clear();
-    stack.clear();
-    stack.push_back(0);
-    while (!stack.empty()) {
-      int i = stack.back();
-      stack.pop_back();
-      order.push_back(i);
-      const RefNode& r = nodes[i];
-      if (r.primitiveCount == 0) {
-        bool neg = (o >> r.axis) & 1;  // basic.cu:180-186: second child first when the direction is negative
-        int nearC = neg ? r.offset : i + 1, farC = neg ? i + 1 : r.offset;
-        stack.push_back(farC);
-        stack.push_back(nearC);
-      }
-    }
+    visit_order(nodes, o, order);
     // before[p]: kept nodes among the first p of the visit order = copy index of the first kept record at or after p
     // (every position has one: leaves are always kept, and a left-out node is followed by its subtree)
     for (int p = 0; p < n; p++) before[p + 1] = before[p] + (keep[order[p]] ? 1 : 0);
@@ -495,11 +502,155 @@ static std::vector<char> pruned_keep(const RefNode* nodes, int n) {
   return keep;
 }
 
-// Full copies (records [0, 8 n)), then the pruned copies (from record 8 n).  Returns the pruned stride.
-static int build_threaded(const RefNode* nodes, int n, std::vector<LtThreadNode>& out) {
+// Traversal tree (LtThreadNode).  By the argument above, applied to every ancestor of a leaf L, the reference reaches
+// L exactly when L's own box is hit, provided L's box lies inside all its ancestors' boxes: which leaves a ray reaches
+// is a property of the leaf boxes alone.  Any tree over the same leaves with containing inner boxes reaches the same
+// ones and changes only the order of the triangle tests; the reference's result is the least (t, rank), rank = the
+// leaf's position in the reference's visit order of the ray's octant (tri_test).  NaN t is never accepted, t == tInit
+// without a hit stays rejected, and an any-hit ray only asks whether some reached triangle is accepted.
+//
+// Whether the reference's leaves allow one: every leaf box inside each of its ancestors' boxes, all bounds finite
+// with lo <= hi (the builder below sorts centroids and sums areas), no primitive linked by two leaves (a rank per
+// primitive), an inner root.  The tie-break table (8 ints per primitive) may take at most as much memory as the
+// threaded copies (16 records per node): a small tree over a huge primitive array keeps the reference's copies.
+static bool leaves_decide_reach(const RefNode* nodes, int n, int primCount) {
+  if (n < 3 || nodes[0].primitiveCount > 0 || (long long)primCount > 16ll * n) return false;
+  // lo, hi of node i: the intersection of its ancestors' boxes
+  std::vector<float> lo((size_t)n * 3, -INFINITY), hi((size_t)n * 3, INFINITY);
+  std::vector<char> linked((size_t)primCount, 0);
+  for (int i = 0; i < n; i++) {  // parents precede their children in the depth-first array
+    const RefNode& r = nodes[i];
+    for (int k = 0; k < 3; k++)
+      if (!(std::isfinite(r.boundsMin[k]) && std::isfinite(r.boundsMax[k]) && r.boundsMin[k] <= r.boundsMax[k]))
+        return false;
+    if (r.primitiveCount > 0) {
+      for (int k = 0; k < 3; k++)
+        if (r.boundsMin[k] < lo[(size_t)i * 3 + k] || r.boundsMax[k] > hi[(size_t)i * 3 + k]) return false;
+      if (linked[r.offset]) return false;
+      linked[r.offset] = 1;
+      continue;
+    }
+    for (int c : {i + 1, r.offset})
+      for (int k = 0; k < 3; k++) {
+        lo[(size_t)c * 3 + k] = std::max(lo[(size_t)i * 3 + k], r.boundsMin[k]);
+        hi[(size_t)c * 3 + k] = std::min(hi[(size_t)i * 3 + k], r.boundsMax[k]);
+      }
+  }
+  return true;
+}
+
+// SAH tree over the reference's leaves, in the reference's depth-first layout.  Each leaf record is copied as it is:
+// its box gates its triangle test, and a multi-primitive leaf's box may be larger than the one triangle it tests.
+// Inner boxes are the exact float min/max of their children, `axis` the split axis (lower centroids in the first
+// child).  Every split is a full sweep over the leaf-box centroids on each axis, minimising
+// SA(first) * leaves(first) + SA(second) * leaves(second).  A full binary tree over the same leaves: n nodes again.
+// Box tests per ray on a stand-in ray stream (tools/threaded_prune_counts.py, profiles/traversal_tree_counts.txt),
+// Cornell box: 10.77 on the reference's pruned copies, 7.30 on this tree's, 6.90 on a PLOC tree's over the primitives.
+static std::vector<RefNode> build_traversal_tree(const RefNode* nodes, int n) {
+  std::vector<int> leaf;  // items: leaf ordinal -> reference node
+  for (int i = 0; i < n; i++)
+    if (nodes[i].primitiveCount > 0) leaf.push_back(i);
+  const int m = (int)leaf.size();
+  std::vector<double> cen((size_t)m * 3);
+  for (int j = 0; j < m; j++)
+    for (int k = 0; k < 3; k++) cen[(size_t)j * 3 + k] = (double)nodes[leaf[j]].boundsMin[k] + nodes[leaf[j]].boundsMax[k];
+  std::vector<int> item(m);
+  for (int j = 0; j < m; j++) item[j] = j;
+  std::vector<RefNode> out((size_t)(2 * m - 1));
+  std::vector<double> secondCost(m);
+  struct Box {
+    float mn[3] = {INFINITY, INFINITY, INFINITY}, mx[3] = {-INFINITY, -INFINITY, -INFINITY};
+    void grow(const RefNode& r) {
+      for (int k = 0; k < 3; k++) {
+        mn[k] = std::min(mn[k], r.boundsMin[k]);
+        mx[k] = std::max(mx[k], r.boundsMax[k]);
+      }
+    }
+    double area() const {
+      double dx = (double)mx[0] - mn[0], dy = (double)mx[1] - mn[1], dz = (double)mx[2] - mn[2];
+      return dx * dy + dy * dz + dz * dx;
+    }
+  };
+  struct Task { int begin, end, parent; };  // parent >= 0: this range is the second child of node `parent`
+  std::vector<Task> todo = {{0, m, -1}};
+  int next = 0;
+  while (!todo.empty()) {
+    const Task tk = todo.back();
+    todo.pop_back();
+    const int idx = next++;
+    if (tk.parent >= 0) out[tk.parent].offset = idx;
+    const int b = tk.begin, e = tk.end;
+    if (e - b == 1) {
+      out[idx] = nodes[leaf[item[b]]];
+      continue;
+    }
+    int bestAxis = 0, bestCut = b + 1;
+    double bestCost = INFINITY;
+    for (int k = 0; k < 3; k++) {
+      std::sort(item.begin() + b, item.begin() + e, [&](int x, int y) {
+        double cx = cen[(size_t)x * 3 + k], cy = cen[(size_t)y * 3 + k];
+        return cx < cy || (cx == cy && x < y);
+      });
+      Box second, first;
+      for (int j = e - 1; j > b; j--) {
+        second.grow(nodes[leaf[item[j]]]);
+        secondCost[j] = second.area() * (e - j);
+      }
+      for (int j = b + 1; j < e; j++) {  // cut j: first child [b, j), second [j, e)
+        first.grow(nodes[leaf[item[j - 1]]]);
+        const double cost = first.area() * (j - b) + secondCost[j];
+        if (cost < bestCost) {
+          bestCost = cost;
+          bestAxis = k;
+          bestCut = j;
+        }
+      }
+    }
+    if (bestAxis != 2)
+      std::sort(item.begin() + b, item.begin() + e, [&](int x, int y) {
+        double cx = cen[(size_t)x * 3 + bestAxis], cy = cen[(size_t)y * 3 + bestAxis];
+        return cx < cy || (cx == cy && x < y);
+      });
+    Box all;
+    for (int j = b; j < e; j++) all.grow(nodes[leaf[item[j]]]);
+    RefNode& nd = out[idx];
+    memset(&nd, 0, sizeof nd);
+    for (int k = 0; k < 3; k++) {
+      nd.boundsMin[k] = all.mn[k];
+      nd.boundsMax[k] = all.mx[k];
+    }
+    nd.axis = (uint8_t)bestAxis;
+    todo.push_back({bestCut, e, idx});  // second child, placed after the whole first subtree
+    todo.push_back({b, bestCut, -1});   // first child: the next node, idx + 1
+  }
+  return out;
+}
+
+// rank[o * primCount + p]: the position of the leaf linking primitive p among the leaves of octant o's reference visit
+// order (the sequence of append_threaded's copy o).  Primitives no leaf links keep 0: they are never tested.
+static std::vector<int> leaf_ranks(const RefNode* nodes, int primCount) {
+  std::vector<int> rank((size_t)8 * primCount, 0), order;
+  for (int o = 0; o < 8; o++) {
+    visit_order(nodes, o, order);
+    int pos = 0;
+    for (int i : order)
+      if (nodes[i].primitiveCount > 0) rank[(size_t)o * primCount + nodes[i].offset] = pos++;
+  }
+  return rank;
+}
+
+// Full copies of the reference tree (records [0, 8 n)), then the pruned copies (from record 8 n): of the traversal
+// tree when the reference's leaves decide reach, with its tie-break table in `rank`; otherwise of the reference tree,
+// and `rank` empty.  Returns the pruned stride.
+static int build_threaded(const RefNode* nodes, int n, int primCount, std::vector<LtThreadNode>& out,
+                          std::vector<int>& rank) {
   out.clear();
+  rank.clear();
   append_threaded(nodes, n, std::vector<char>(n, 1), out);
-  return append_threaded(nodes, n, pruned_keep(nodes, n), out);
+  if (!leaves_decide_reach(nodes, n, primCount)) return append_threaded(nodes, n, pruned_keep(nodes, n), out);
+  const std::vector<RefNode> trav = build_traversal_tree(nodes, n);
+  rank = leaf_ranks(nodes, primCount);
+  return append_threaded(trav.data(), (int)trav.size(), pruned_keep(trav.data(), (int)trav.size()), out);
 }
 
 static int debug_tree_arg(const void* nodes, uint64_t node_bytes, const char* who, int* n) {
@@ -532,6 +683,36 @@ extern "C" int lt_debug_build_threaded_pruned(const void* nodes, uint64_t node_b
   *out_stride = append_threaded((const RefNode*)nodes, n, pruned_keep((const RefNode*)nodes, n), out);
   if (out_records) memcpy(out_records, out.data(), out.size() * sizeof(LtThreadNode));
   return LT_OK;
+}
+
+// What lt_scene_upload builds for a small tree: out_records (16 n records of room) receives the full copies and then the
+// pruned ones, skip links as uploaded (absolute, from record 8 n); out_rank (8 x prim_count ints of room) the
+// tie-break table when *out_traversal == 1, i.e. when the pruned copies are a traversal tree.
+extern "C" int lt_debug_build_traversal_tree(const void* nodes, uint64_t node_bytes, int32_t prim_count,
+                                             void* out_records, int32_t* out_stride, int32_t* out_rank,
+                                             int32_t* out_traversal) {
+  const char* who = "lt_debug_build_traversal_tree";
+  int n = 0;
+  if (!out_records || !out_stride || !out_rank || !out_traversal || prim_count < 1)
+    return fail(nullptr, LT_ERR_INVALID, std::string(who) + ": bad arguments");
+  if (int rc = debug_tree_arg(nodes, node_bytes, who, &n)) return rc;
+  const RefNode* r = (const RefNode*)nodes;
+  for (int i = 0; i < n; i++)
+    if (r[i].primitiveCount > 0 && r[i].offset >= prim_count)
+      return fail(nullptr, LT_ERR_INVALID, std::string(who) + ": leaf primitivesOffset out of range");
+  std::vector<LtThreadNode> out;
+  std::vector<int> rank;
+  *out_stride = build_threaded(r, n, prim_count, out, rank);
+  *out_traversal = rank.empty() ? 0 : 1;
+  memcpy(out_records, out.data(), out.size() * sizeof(LtThreadNode));
+  if (!rank.empty()) memcpy(out_rank, rank.data(), rank.size() * sizeof(int));
+  return LT_OK;
+}
+
+extern "C" int lt_debug_scene_traversal_tree(const lt_scene* scene) {
+  if (!scene) return fail(nullptr, LT_ERR_INVALID, "lt_debug_scene_traversal_tree: scene is NULL");
+  if (!scene->parts.empty()) scene = scene->parts[0];
+  return scene->dev.rank != nullptr ? 1 : 0;
 }
 
 // Where trav_begin_threaded starts the rays that may use pruned records: the pruned copies of dThread, or (no host-built
@@ -577,13 +758,18 @@ static int finish_scene(lt_ctx* ctx, lt_scene* s, int nNodes, int nPrims, int nM
   if (e == cudaSuccess && copies == LT_TREE_HOST_THREADED) {
     std::vector<RefNode> hNodes((size_t)nNodes);
     std::vector<LtThreadNode> hThread;
+    std::vector<int> hRank;
     A(cudaMemcpyAsync(hNodes.data(), s->dNodes, sizeof(RefNode) * (size_t)nNodes, cudaMemcpyDeviceToHost, st));
     A(cudaStreamSynchronize(st));
     if (e == cudaSuccess) {
-      s->threadStride = build_threaded(hNodes.data(), nNodes, hThread);
+      s->threadStride = build_threaded(hNodes.data(), nNodes, nPrims, hThread, hRank);
       A(cudaMalloc(&s->dThread, sizeof(LtThreadNode) * hThread.size()));
       A(cudaMemcpyAsync(s->dThread, hThread.data(), sizeof(LtThreadNode) * hThread.size(), cudaMemcpyHostToDevice, st));
-      A(cudaStreamSynchronize(st));  // hThread is pageable and goes out of scope
+      if (!hRank.empty()) {
+        A(cudaMalloc(&s->dRank, sizeof(int) * hRank.size()));
+        A(cudaMemcpyAsync(s->dRank, hRank.data(), sizeof(int) * hRank.size(), cudaMemcpyHostToDevice, st));
+      }
+      A(cudaStreamSynchronize(st));  // hThread and hRank are pageable and go out of scope
     }
   }
   // large trees: the threaded copies are built on the device and used by coherent-ray launches only (plan_tree)
@@ -623,6 +809,7 @@ static int finish_scene(lt_ctx* ctx, lt_scene* s, int nNodes, int nPrims, int nM
   d.primCount = nPrims;
   d.matCount = nMats;
   d.tnodes = s->dThread;
+  d.rank = s->dRank;
   d.tnodesCoherent = s->dThreadBig;
   set_pruned_copies(s, false);
   return LT_OK;

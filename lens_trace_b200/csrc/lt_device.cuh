@@ -66,9 +66,12 @@ __device__ __forceinline__ bool slab(float lox, float hix, float loy, float hiy,
 }
 
 // intersectTriangle, basic.cu:93-134, on the pre-subtracted record.  Returns true when the hit
-// record was replaced (strict t < best, no t > 0 test -- both as in the reference).
+// record was replaced (strict t < best, no t > 0 test -- both as in the reference).  The reference thus keeps the
+// least (t, position in its visit order): a walk in another order (the traversal tree's pruned copies) passes
+// rank = LtSceneDev::rank and row = octant * primCount, and a t equal to the best one replaces it when its rank is
+// lower.  Walks in the reference's order pass NULL: there the ranks rise along the walk and the tie-break never fires.
 __device__ __forceinline__ bool tri_test(const LtTri* __restrict__ tris, int prim, const Ray& r, float epsThr,
-                                         Hit& h) {
+                                         Hit& h, const int* __restrict__ rank, int row = 0) {
   const float4* tp = reinterpret_cast<const float4*>(tris + prim);
   float4 q0 = __ldg(tp), q1 = __ldg(tp + 1), q2 = __ldg(tp + 2);
   float ax = q0.x, ay = q0.y, az = q0.z;
@@ -89,7 +92,10 @@ __device__ __forceinline__ bool tri_test(const LtTri* __restrict__ tris, int pri
   float v = FMUL(dot3z(r.dx, r.dy, r.dz, qx, qy, qz), inv);
   if (v < 0.0f || FADD(u, v) > 1.0f) return false;
   float t = FMUL(dot3z(e2x, e2y, e2z, qx, qy, qz), inv);
-  if (t < h.t) {
+  // t == tInit without a hit stays rejected (h.hit), NaN fails both comparisons, and -0 == +0 is a tie
+  if (t < h.t ||
+      (rank != nullptr && __builtin_expect(t == h.t && h.hit != 0, 0) &&
+       __ldg(rank + row + prim) < __ldg(rank + row + h.prim))) {
     h.t = t;
     h.u = u;
     h.v = v;
@@ -282,7 +288,7 @@ __device__ __forceinline__ bool trav_test(Trav& t, const LtSceneDev& sc, const i
   for (int i = 0; i < n; i++) {
     int prim = list[i * LT_THREAD_STRIDE];
     if (STATS) cnt.triTests++;
-    if (tri_test(sc.tris, prim, t.r, epsThr, t.h)) {
+    if (tri_test(sc.tris, prim, t.r, epsThr, t.h, nullptr)) {
       t.h.prim = prim;
       t.h.hit = 1;
       if (t.anyHit) {
@@ -380,7 +386,7 @@ __device__ __forceinline__ bool trav_iter_lean(Trav& t, const LtSceneDev& sc, un
     int prim = lds32(fifoAddr + ((unsigned)(t.qHead & (LT_MAX_BATCH - 1)) * LT_LEVEL_BYTES));
     t.qHead++;
     if (STATS) cnt.triTests++;
-    if (tri_test(sc.tris, prim, t.r, epsThr, t.h)) {
+    if (tri_test(sc.tris, prim, t.r, epsThr, t.h, nullptr)) {
       t.h.prim = prim;
       t.h.hit = 1;
       if (t.anyHit) {
@@ -461,19 +467,18 @@ __device__ __forceinline__ void trav_threaded_nodes(Trav& t, const LtThreadNode*
 // steps of kLeanNodeSteps
 constexpr int kThreadedNodeSteps = 2 * kLeanNodeSteps;
 constexpr int kThreadedTriTests = kLeanTriTests;
-__device__ __forceinline__ bool trav_iter_threaded(Trav& t, const LtThreadNode* __restrict__ tn,
-                                                   const LtTri* __restrict__ tris, unsigned fifoAddr, float epsThr,
+__device__ __forceinline__ bool trav_iter_threaded(Trav& t, const LtSceneDev& sc, unsigned fifoAddr, float epsThr,
                                                    int nodeSteps, int triTests) {
   // rays change only between iterations, so which slab form the warp runs is decided once per iteration
   const bool exact = __any_sync(__activemask(), (t.negMask & LT_EXACT_SLAB) != 0u);
   const int maxSteps = min(nodeSteps, LT_MAX_BATCH - (t.qTail - t.qHead));
   const int notIgnore = ~t.ignore;  // a leaf's link is ~primitivesOffset
-  if (exact) trav_threaded_nodes<true>(t, tn, fifoAddr, maxSteps, notIgnore);
-  else trav_threaded_nodes<false>(t, tn, fifoAddr, maxSteps, notIgnore);
+  if (exact) trav_threaded_nodes<true>(t, sc.tnodes, fifoAddr, maxSteps, notIgnore);
+  else trav_threaded_nodes<false>(t, sc.tnodes, fifoAddr, maxSteps, notIgnore);
   for (int k = 0; k < triTests && t.qHead != t.qTail; k++) {
     int prim = lds32(fifoAddr + ((unsigned)(t.qHead & (LT_MAX_BATCH - 1)) * LT_LEVEL_BYTES));
     t.qHead++;
-    if (tri_test(tris, prim, t.r, epsThr, t.h)) {
+    if (tri_test(sc.tris, prim, t.r, epsThr, t.h, sc.rank, (int)(t.negMask & 7u) * sc.primCount)) {
       t.h.prim = prim;
       t.h.hit = 1;
       if (t.anyHit) {
@@ -555,7 +560,7 @@ __device__ __forceinline__ void trav_step_cull(Trav& t, const LtSceneDev& sc, in
     int prim = ~t.cur;
     if (prim != t.ignore) {
       if (STATS) cnt.triTests++;
-      if (tri_test(sc.tris, prim, t.r, epsThr, t.h)) {
+      if (tri_test(sc.tris, prim, t.r, epsThr, t.h, nullptr)) {
         t.h.prim = prim;
         t.h.hit = 1;
       }
@@ -596,7 +601,7 @@ __device__ __forceinline__ void trace(Trav& t, const LtSceneDev& sc, int ignore,
   if (!STATS && sc.tnodes != nullptr) {  // small scene: stackless traversal of the threaded tree, same tests
     trav_begin_threaded(t, sc, ignore, tInit, anyHit);
     const unsigned fifoAddr = (unsigned)__cvta_generic_to_shared(list);
-    while (!trav_iter_threaded(t, sc.tnodes, sc.tris, fifoAddr, epsThr, LT_MAX_BATCH, LT_MAX_BATCH)) {
+    while (!trav_iter_threaded(t, sc, fifoAddr, epsThr, LT_MAX_BATCH, LT_MAX_BATCH)) {
     }
     return;
   }

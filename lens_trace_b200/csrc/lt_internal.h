@@ -165,6 +165,7 @@ struct lt_scene {
   LtTri* dTris = nullptr;
   LtThreadNode* dThread = nullptr;  // 8 octant copies in visit order, then 8 pruned ones, small scenes only
   int threadStride = 0;             // records per pruned copy
+  int* dRank = nullptr;             // LtSceneDev::rank, when the pruned copies are a traversal tree
   LtThreadNode* dThreadBig = nullptr;  // the same for a large scene, built on the device, for coherent-ray launches
   LtSceneDev dev = {};
 };

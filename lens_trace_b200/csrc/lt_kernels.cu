@@ -237,7 +237,7 @@ __global__ void __launch_bounds__(LT_BLOCK) k_path(LtSceneDev sc, LtLaunch L, fl
       if (waiting && __popc(active) < kPathRefillLanes) break;
       if (traversing) {
         if (threaded) {
-          traversing = !trav_iter_threaded(t, sc.tnodes, sc.tris, fifoAddr, pc.epsThr, kThreadedNodeSteps, kThreadedTriTests);
+          traversing = !trav_iter_threaded(t, sc, fifoAddr, pc.epsThr, kThreadedNodeSteps, kThreadedTriTests);
         } else {
           int n = trav_collect<STATS>(t, sc, stk, list, LT_MAX_BATCH, cnt);
           trav_test<STATS>(t, sc, list, n, pc.epsThr, cnt);

@@ -381,7 +381,7 @@ __global__ void __launch_bounds__(WF_BLOCK) __maxnreg__(STATS ? 64 : 56)
     if (has) {
       bool finished;
       if (THREADED) {
-        finished = trav_iter_threaded(t, sc.tnodes, sc.tris, fifoAddr, epsThr, kThreadedNodeSteps, kThreadedTriTests);
+        finished = trav_iter_threaded(t, sc, fifoAddr, epsThr, kThreadedNodeSteps, kThreadedTriTests);
       } else if (cull && !t.anyHit) {  // a round holds one kind of ray, so this does not split warps
         for (int k = 0; k < 2 * kLeanNodeSteps && t.cur != LT_DONE; k++)
           trav_step_cull<STATS>(t, sc, stk, tstk, epsThr, cnt);

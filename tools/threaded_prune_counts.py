@@ -5,7 +5,9 @@ parameters).  Rays: the camera rays of the default camera at W x H and, from eve
 uniformly sampled direction of the hemisphere around the shading normal (seeded) -- a stand-in for the GI kernel's
 ray stream, which the library does not expose.  For the real stream, the oracle's own count of the reference's box
 tests (full sequences, root included) is printed beside it.  Rays with a zero or non-finite reciprocal walk the full
-copies on the device and are counted there.
+copies on the device and are counted there.  Beside them: the pruned copies of the traversal tree lt_scene_upload
+builds over the reference's leaves (lt_debug_build_traversal_tree, SAH), and those of a PLOC tree over the primitives
+(the NumPy restatement of tests/test_ploc_builder.py), which reach the same triangles.
     python tools/threaded_prune_counts.py [model] [W H]"""
 import os
 import sys
@@ -17,6 +19,7 @@ import lt_oracle as O  # noqa: E402
 import util  # noqa: E402
 from lens_trace_b200 import capi, layouts as L  # noqa: E402
 from test_threaded_prune import _walk  # noqa: E402
+from test_ploc_builder import emit, ploc_tree  # noqa: E402
 
 model = sys.argv[1] if len(sys.argv) > 1 else "cornell_box"
 w = int(sys.argv[2]) if len(sys.argv) > 2 else 480
@@ -60,6 +63,15 @@ print("%s: %d nodes, %d records per pruned copy; %d rays (%d camera, %d bounce),
     model, len(sb.nodes), pruned.shape[1], len(O3), w * h, int(m.sum()), int((~pruned_ok).sum())))
 print("box tests per ray, root excluded: full copies %.2f, pruned copies %.2f (%+.1f %%)" % (
     tf.mean() - 1, tp.mean() - 1, 100.0 * (tp.mean() - tf.mean()) / (tf.mean() - 1)))
+trav = capi.build_traversal_tree(sb.nodes, len(sb.prims))
+assert trav["traversal"]
+ploc_sb, _ = emit(ploc_tree(sb.prims), sb.prims, sb.materials)
+ploc = capi.build_threaded_pruned(ploc_sb.nodes)
+for name, T in (("traversal tree (SAH over the leaves)", trav["pruned"]), ("PLOC tree over the primitives", ploc)):
+    tt = tf.copy()
+    _, _, tt[pruned_ok] = _walk(T, O3[pruned_ok], INV[pruned_ok])
+    print("  %s: %d records per pruned copy, %.2f box tests per ray (%+.1f %% against the reference's pruned copies)"
+          % (name, T.shape[1], tt.mean() - 1, 100.0 * (tt.mean() - tp.mean()) / (tp.mean() - 1)))
 _, st = O.render(L.KERNEL_GI, sb, util.default_camera(0.0, 0), w, h, max_ray_depth=4, with_stats=True, threads=0)
 print("GI kernel, frame 0, depth 4 (oracle): %d rays, %.2f box tests per ray on the full sequences, root included" % (
     st.rays, st.nodeTests / st.rays))
