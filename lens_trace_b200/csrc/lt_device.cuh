@@ -892,6 +892,13 @@ __device__ __forceinline__ void sample_hemisphere(float u1, float u2, const floa
   dir[3] = hy;
 }
 
+// dot(previousNormal (w = 1), direction (w = hemisphere.y)), global_illumination.cl:321: what a light hit of the
+// extension ray `dir` (w = hemisphere.y) drawn at the shading point of normal `nrm` adds per depth.  Every input is
+// known when the ray is drawn, so the path carries this one number to the hit instead of the normal and direction.
+__device__ __forceinline__ float light_hit_cos(const float nrm[3], const float dir[4]) {
+  return FADD(FADD(FADD(FMUL(nrm[0], dir[0]), FMUL(nrm[1], dir[1])), FMUL(nrm[2], dir[2])), FMUL(1.0f, dir[3]));
+}
+
 enum PathStage { ST_PRIMARY = 0, ST_SHADOW_DIRECT = 1, ST_EXTENSION = 2, ST_SHADOW_EXT = 3 };
 
 // ------------------------------------------------------------------------------------------------
@@ -907,6 +914,12 @@ struct PathConsts {
   bool foldLightHits;  // see shade_step: a light hit's remaining depths are accumulated without retracing the ray
 };
 
+// Counting launches trace what the reference traces, unless LT_FLAG_STATS_TRACED asks for the counts of what the
+// exact pipelines really trace.  Host side too: a launch that folds light hits has homogeneous wavefront rounds.
+__host__ __device__ __forceinline__ bool lt_fold_light_hits(int flags) {
+  return !(flags & LT_DEV_FLAG_STATS) || (flags & LT_DEV_FLAG_STATS_TRACED);
+}
+
 __device__ __forceinline__ PathConsts path_consts(const LtLaunch& L) {
   PathConsts pc;
   pc.tInit = lt_tinit(L.kernel);
@@ -915,16 +928,14 @@ __device__ __forceinline__ PathConsts path_consts(const LtLaunch& L) {
   pc.whiteOnLight = (L.kernel == LT_DEV_KERNEL_ACCUMULATOR);
   pc.samplesPerFrame = (L.kernel == LT_DEV_KERNEL_LIGHTING25 || L.kernel == LT_DEV_KERNEL_GI25) ? 25 : 1;
   pc.maxDepth = L.maxRayDepth > 0 ? L.maxRayDepth : 16;
-  // counting launches trace what the reference traces, unless LT_FLAG_STATS_TRACED asks for the counts of what the
-  // exact pipelines really trace
-  pc.foldLightHits = !(L.flags & LT_DEV_FLAG_STATS) || (L.flags & LT_DEV_FLAG_STATS_TRACED);
+  pc.foldLightHits = lt_fold_light_hits(L.flags);
   return pc;
 }
 
 struct PathState {
   float nrm[3], diffuse[3];
   float direct[3], indirect[3];
-  float extW;   // w of the extension direction (= hemisphere.y, global_illumination.cl:239)
+  float dLight;  // light_hit_cos of the extension ray: what a light hit at its end adds per depth
   int hitPrim;  // primitive the current shading point lies on (= previousPrimitive of the reference)
   int depth;
   int stage;    // PathStage
@@ -957,13 +968,12 @@ __device__ __forceinline__ bool shade_step(const LtSceneDev& sc, const PathConst
         ps.direct[0] = ps.direct[1] = ps.direct[2] = 1.0f;
         sampleDone = true;
       } else {
-        // dot(previousNormal (w = 1), direction (w = hemisphere.y)), global_illumination.cl:321.
+        // d = light_hit_cos of this ray, computed where it was drawn.
         // The reference does not advance the ray, so it traces the same ray again at the next depth, finds the same
         // hit (the hit is a function of the ray alone) and lands here again, until maxDepth.  Those traversals change
         // nothing but the depth: the remaining terms 1/(depth+1) * d are added here, in the same order, without
         // tracing (the counting launches still retrace, so that their counts are the reference's).
-        const float d = FADD(FADD(FADD(FMUL(ps.nrm[0], r.dx), FMUL(ps.nrm[1], r.dy)), FMUL(ps.nrm[2], r.dz)),
-                             FMUL(1.0f, ps.extW));
+        const float d = ps.dLight;
         do {
           float w = (float)__ddiv_rn(1.0, (double)(ps.depth + 1));
           float c = FMUL(FMUL(w, 1.0f), d);
@@ -1044,7 +1054,7 @@ __device__ __forceinline__ bool shade_step(const LtSceneDev& sc, const PathConst
     float dir[4];
     sample_hemisphere(rA, rB, ps.nrm, dir);
     r.dx = dir[0]; r.dy = dir[1]; r.dz = dir[2];  // origin stays the shaded position
-    ps.extW = dir[3];
+    ps.dLight = light_hit_cos(ps.nrm, dir);
     ignore = ps.hitPrim;
     ps.stage = ST_EXTENSION;
   } else if (retrace) {

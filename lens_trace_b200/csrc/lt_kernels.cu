@@ -177,7 +177,7 @@ __global__ void __launch_bounds__(LT_BLOCK) k_path(LtSceneDev sc, LtLaunch L, fl
   PathState ps;
   ps.nrm[0] = ps.nrm[1] = ps.nrm[2] = 0.0f;
   ps.diffuse[0] = ps.diffuse[1] = ps.diffuse[2] = 0.0f;
-  ps.extW = 0.0f;
+  ps.dLight = 0.0f;
   ps.hitPrim = 0;
   ps.depth = 0;
   path_reset(ps);

@@ -12,8 +12,12 @@
 //
 // In a round all rays are of one kind (all primary, all shadow, all extension), shading code runs on
 // dense arrays, and the running mean is applied in frame order, so results are bit-identical to
-// k_path's.  Between rounds a path's state travels in its queue entry, beside its ray (40 B payload), so every load
+// k_path's.  Between rounds a path's state travels in its queue entry, beside its ray, so every load
 // of a queue entry is indexed by its slot and can be issued at once.
+// Round 1 holds the first shadow rays of the paths, then extension and shadow rounds alternate (WfRound).  The
+// shade kernel is compiled for each kind of round and loads only what that kind reads: a shadow entry its ray,
+// shading normal and colours, an extension entry its hit, colours and one float (dLight).  Counting launches that
+// retrace light hits mix extension rays into shadow rounds; they keep the full entries (WF_GENERIC).
 #include "lt_internal.h"
 #include "lt_device.cuh"
 
@@ -31,16 +35,30 @@ struct LtWfBuffers {
   // Path state of the queue entry (WfPayload), indexed like the rays: the shade kernel loads it in queue order
   // together with the ray and the hit instead of by path id after them.  Stage and depth travel in the path word,
   // hitPrim is the ray's ignore index.
-  float4* payA[2];    // nrm.xyz of the shading point, then bits(material index) for a shadow ray / extW for an extension ray
+  float4* payA[2];    // nrm.xyz of the shading point, then bits(material index) for a shadow ray / dLight for an
+                      // extension ray (WF_GENERIC); other launches keep only dLight of an extension ray: wf_dlight
   float4* payB[2];    // direct.rgb, indirect.r
   float2* payC[2];    // indirect.gb
-  float4* hits;       // t, u, v, bits(prim | hit << 31), indexed like the current queue
+  float4* hits;       // t, u, v, bits(prim | hit << 31), indexed like the current queue; other launches than
+                      // WF_GENERIC keep only the last word of a shadow ray's hit: wf_hit_words
   int* counts;        // [2q], [2q+1] sizes of the front and the back region of queue q (one 64-bit word per queue, so
                       // that one atomic reserves both), [4] trace work counter.  Rays that need the select-chain
                       // slab test (a zero direction component) are appended from the END of the queue, so they
                       // share warps with each other and not with the ordinary rays
   int capacity;       // entries per queue
 };
+
+// The kind of a round, which decides what its queue entries hold and what the shade kernel loads of them.
+// WF_GENERIC: every entry holds its full payload and its full hit record (rounds that may mix kinds).
+// WF_FIRST_SHADOW: round 1, the shadow rays k_wf_primary emits; direct and indirect are still zero, so the entries
+// hold no payB / payC.  WF_SHADOW: the shadow rays of later bounces.  WF_EXTENSION: extension rays; their entries
+// hold no payA but dLight.  In the last three a shadow ray's hit is one word.
+enum WfRound { WF_GENERIC, WF_FIRST_SHADOW, WF_SHADOW, WF_EXTENSION };
+
+// A round holds either shadow or extension entries, never both, so dLight and the shadow hit words can be dense
+// arrays over the start of the buffers whose float4 form the other kind uses: the workspace does not grow.
+__device__ __forceinline__ float* wf_dlight(const LtWfBuffers& B, int q) { return reinterpret_cast<float*>(B.payA[q]); }
+__device__ __forceinline__ int* wf_hit_words(const LtWfBuffers& B) { return reinterpret_cast<int*>(B.hits); }
 
 #define WF_PATH_BITS 25  // a batch holds at most 2^25 paths (lt_capi.cu caps it)
 __device__ __forceinline__ int wf_pack_path(int path, int stage, int depth) {
@@ -71,8 +89,8 @@ __device__ __forceinline__ bool ray_is_degenerate(const Ray& r) {
 }
 
 // What the next shading of a queue entry reads of its path, beside the ray (LtWfBuffers::payA/B/C).  A shadow ray's
-// shading reads the diffuse colour of its shading point, an extension ray's the w of its direction: one word holds
-// the material index (the diffuse colour is a load from the small materials table) or extW.
+// shading reads the normal and the diffuse colour of its shading point, an extension ray's only dLight: one word
+// holds the material index (the diffuse colour is a load from the small materials table) or dLight.
 struct WfPayload {
   float4 a, b;
   float2 c;
@@ -86,10 +104,27 @@ __device__ __forceinline__ WfPayload wf_payload(const PathState& ps, float sel) 
   return pl;
 }
 
+// the stores of one queue entry, for a round of kind OUT
+template <int OUT>
+__device__ __forceinline__ void queue_store(const LtWfBuffers& B, int dst, int slot, const Ray& r, float tStart,
+                                            int ignore, bool anyHit, int path, const WfPayload& pl) {
+  B.rayO[dst][slot] = make_float4(r.ox, r.oy, r.oz, tStart);
+  B.rayD[dst][slot] = make_float4(r.dx, r.dy, r.dz,
+                                  __int_as_float((int)((unsigned)(ignore + 1) | (anyHit ? 0x80000000u : 0u))));
+  B.rayPath[dst][slot] = path;
+  if (OUT == WF_EXTENSION) wf_dlight(B, dst)[slot] = pl.a.w;
+  else B.payA[dst][slot] = pl.a;
+  if (OUT != WF_FIRST_SHADOW) {
+    B.payB[dst][slot] = pl.b;
+    B.payC[dst][slot] = pl.c;
+  }
+}
+
 // Block-aggregated append of this thread's ray (if emit) to queue `dst`; every thread of the block calls it the
 // same number of times.  One global atomic per block and call -- on a packed 64-bit counter (front count in the
 // low word, back count in the high word) -- instead of up to two per warp: ncu attributed 31 % of the shade
 // kernel's stall samples to the wait for those same-address atomics.
+template <int OUT>
 __device__ __forceinline__ void queue_append(const LtWfBuffers& B, int dst, bool emit, const Ray& r, float tStart,
                                              int ignore, bool anyHit, int path, const WfPayload& pl, unsigned lane) {
   __shared__ unsigned s_warpCount[WF_BLOCK / 32];  // front | back << 16 of each warp
@@ -116,20 +151,15 @@ __device__ __forceinline__ void queue_append(const LtWfBuffers& B, int dst, bool
     int slot;
     if (front) slot = (int)(unsigned)base + (int)(before & 0xffffu) + __popc(fm & ((1u << lane) - 1u));
     else slot = B.capacity - 1 - ((int)(unsigned)(base >> 32) + (int)(before >> 16) + __popc(bm & ((1u << lane) - 1u)));
-    B.rayO[dst][slot] = make_float4(r.ox, r.oy, r.oz, tStart);
-    B.rayD[dst][slot] = make_float4(r.dx, r.dy, r.dz,
-                                    __int_as_float((int)((unsigned)(ignore + 1) | (anyHit ? 0x80000000u : 0u))));
-    B.rayPath[dst][slot] = path;
-    B.payA[dst][slot] = pl.a;
-    B.payB[dst][slot] = pl.b;
-    B.payC[dst][slot] = pl.c;
+    queue_store<OUT>(B, dst, slot, r, tStart, ignore, anyHit, path, pl);
   }
 }
 
-// warp-aggregated form (no block barrier) for the primary round, where most warps of a sparse view emit nothing
+// warp-aggregated form (no block barrier) for the primary round, where most warps of a sparse view emit nothing;
+// out: WF_FIRST_SHADOW or WF_GENERIC
 __device__ __forceinline__ void queue_append_warp(const LtWfBuffers& B, int dst, bool emit, const Ray& r, float tStart,
                                                   int ignore, bool anyHit, int path, const WfPayload& pl,
-                                                  unsigned lane) {
+                                                  unsigned lane, int out) {
   bool back = emit && ray_is_degenerate(r);
   bool front = emit && !back;
   unsigned fm = __ballot_sync(0xffffffffu, front), bm = __ballot_sync(0xffffffffu, back);
@@ -143,13 +173,8 @@ __device__ __forceinline__ void queue_append_warp(const LtWfBuffers& B, int dst,
     int slot;
     if (front) slot = (int)(unsigned)base + __popc(fm & ((1u << lane) - 1u));
     else slot = B.capacity - 1 - ((int)(unsigned)(base >> 32) + __popc(bm & ((1u << lane) - 1u)));
-    B.rayO[dst][slot] = make_float4(r.ox, r.oy, r.oz, tStart);
-    B.rayD[dst][slot] = make_float4(r.dx, r.dy, r.dz,
-                                    __int_as_float((int)((unsigned)(ignore + 1) | (anyHit ? 0x80000000u : 0u))));
-    B.rayPath[dst][slot] = path;
-    B.payA[dst][slot] = pl.a;
-    B.payB[dst][slot] = pl.b;
-    B.payC[dst][slot] = pl.c;
+    if (out == WF_FIRST_SHADOW) queue_store<WF_FIRST_SHADOW>(B, dst, slot, r, tStart, ignore, anyHit, path, pl);
+    else queue_store<WF_GENERIC>(B, dst, slot, r, tStart, ignore, anyHit, path, pl);
   }
 }
 
@@ -232,9 +257,11 @@ __global__ void __launch_bounds__(WF_BLOCK) k_wf_primary_trace(LtSceneDev sc, Lt
 // primaryHits != nullptr: the per-pixel records of k_wf_primary_trace replace the trace (exact, uncounted launches)
 // P.alive != nullptr: only the alive pixels get paths (nf frames x aliveCount pixels, enumerated through the list);
 // the path id stays frame * pixels + pixel, so nothing downstream changes.
+// out: the kind of round 1 (WF_FIRST_SHADOW, or WF_GENERIC), which decides what its entries hold
 template <bool STATS>
 __global__ void __launch_bounds__(WF_BLOCK) k_wf_primary(LtSceneDev sc, LtLaunch L, LtWfBuffers B, int nf,
-                                                         int pixels, int sample, LtCounters* gcnt, LtWfPrimary P) {
+                                                         int pixels, int sample, LtCounters* gcnt, LtWfPrimary P,
+                                                         int out) {
   LT_SMEM_POINTERS(sc)
   const float4* __restrict__ primaryHits = P.hits;
   const bool cull = (L.flags & LT_DEV_FLAG_CULL) != 0;  // closest-hit rays skip subtrees behind the current hit
@@ -280,7 +307,7 @@ __global__ void __launch_bounds__(WF_BLOCK) k_wf_primary(LtSceneDev sc, LtLaunch
       PathState ps;
       ps.nrm[0] = ps.nrm[1] = ps.nrm[2] = 0.0f;
       ps.diffuse[0] = ps.diffuse[1] = ps.diffuse[2] = 0.0f;
-      ps.extW = 0.0f;
+      ps.dLight = 0.0f;
       ps.hitPrim = 0;
       ps.depth = 0;
       path_reset(ps);
@@ -301,7 +328,7 @@ __global__ void __launch_bounds__(WF_BLOCK) k_wf_primary(LtSceneDev sc, LtLaunch
         packed = wf_pack_path((int)p, ps.stage, ps.depth);
       }
     }
-    queue_append_warp(B, 0, emit, t.r, tStart, ignore, anyHit, packed, pl, lane);
+    queue_append_warp(B, 0, emit, t.r, tStart, ignore, anyHit, packed, pl, lane, out);
   }
   if (STATS) flush_counters(gcnt, cnt);
 }
@@ -317,10 +344,13 @@ __global__ void k_wf_reset(LtWfBuffers B) {
 // Exact variants: at most 56 registers, so that one block of the other batch's shade kernel (64 registers) fits on an
 // SM beside 8 trace blocks.  Left to itself ptxas gives the stack variant 64 registers (no spill instead of 4 bytes),
 // and the 1M-triangle GI step then takes 42.7 instead of 42.0-42.4 ms (B200, 1000 W power limit).
+// hitWords: wf_hit_words(B) on a WF_FIRST_SHADOW or WF_SHADOW round, whose rays store only the last word of their hit;
+// nullptr on the others, whose rays store the full record.  (A counting launch traces its shadow rays as closest-hit
+// rays, so the round decides this, not the ray.)
 template <bool STATS, bool THREADED>
 __global__ void __launch_bounds__(WF_BLOCK) __maxnreg__(STATS ? 64 : 56)
     k_wf_trace(LtSceneDev sc, LtLaunch L, LtWfBuffers B, int q, LtCounters* gcnt, const float4* __restrict__ rayO,
-               const float4* __restrict__ rayD) {
+               const float4* __restrict__ rayD, int* __restrict__ hitWords) {
   extern __shared__ int smemStack[];
   int* stk = smemStack + threadIdx.x;
   int* list = smemStack + (THREADED ? 0 : lt_stack_levels(sc) * LT_BLOCK) + threadIdx.x;
@@ -367,7 +397,8 @@ __global__ void __launch_bounds__(WF_BLOCK) __maxnreg__(STATS ? 64 : 56)
           else trav_begin<STATS>(t, sc, (int)(bits & 0x7fffffffu) - 1, o.w, (bits >> 31) != 0u, cnt);
           entry = idx;
           if (t.cur == LT_DONE) {  // missed the root box: finished already
-            B.hits[idx] = make_float4(t.h.t, 0.0f, 0.0f, __int_as_float(0));
+            if (hitWords) hitWords[idx] = 0;
+            else B.hits[idx] = make_float4(t.h.t, 0.0f, 0.0f, __int_as_float(0));
             entry = -1;
           }
         }
@@ -390,8 +421,9 @@ __global__ void __launch_bounds__(WF_BLOCK) __maxnreg__(STATS ? 64 : 56)
         finished = trav_iter_lean<STATS>(t, sc, stkAddr, fifoAddr, epsThr, kLeanNodeSteps, kLeanTriTests, cnt);
       }
       if (finished) {
-        B.hits[entry] = make_float4(t.h.t, t.h.u, t.h.v,
-                                    __int_as_float((int)((unsigned)t.h.prim | (t.h.hit ? 0x80000000u : 0u))));
+        const int word = (int)((unsigned)t.h.prim | (t.h.hit ? 0x80000000u : 0u));
+        if (hitWords) hitWords[entry] = word;
+        else B.hits[entry] = make_float4(t.h.t, t.h.u, t.h.v, __int_as_float(word));
         entry = -1;
       }
     }
@@ -404,10 +436,17 @@ __global__ void __launch_bounds__(WF_BLOCK) __maxnreg__(STATS ? 64 : 56)
 // with a run-time index the compiler copies the pointer arrays of the by-value struct to local memory and every
 // queue access starts with a dependent LDL.  Registers sized for 8 resident blocks (<= 64): measured against 10 and
 // 12 -- the kernel waits on dependent loads, and registers buy it more loads in flight per thread than warps do.
-template <int Q>
+// K (WfRound) is the kind of the round: it fixes the stage of every entry and which arrays are loaded.  A shadow
+// result reads ray, hit word, payA and (after the first bounce) payB / payC; an extension result reads neither its ray
+// nor the normal: a surface hit rebuilds the shading point from the hit, a light hit reads dLight, a miss only
+// finishes the sample.
+template <int Q, int K>
 __global__ void __launch_bounds__(WF_BLOCK, 8) k_wf_shade(LtSceneDev sc, LtLaunch L, LtWfBuffers B, int pixels,
                                                           int frame0, int sample, LtWfPrimary P) {
   constexpr int q = Q;
+  constexpr bool generic = K == WF_GENERIC, extension = K == WF_EXTENSION;
+  // the kind of the round that consumes what this one appends
+  constexpr int OUT = generic ? WF_GENERIC : (extension ? WF_SHADOW : WF_EXTENSION);
   const PathConsts pc = path_consts(L);
   const int nFront = B.counts[2 * q];
   const int n = nFront + B.counts[2 * q + 1];
@@ -426,9 +465,22 @@ __global__ void __launch_bounds__(WF_BLOCK, 8) k_wf_shade(LtSceneDev sc, LtLaunc
     if (valid) {
       const int word = B.rayPath[q][i];
       path = word & ((1 << WF_PATH_BITS) - 1);
-      float4 o = B.rayO[q][i], d = B.rayD[q][i], hv = B.hits[i];
-      const float4 pa = B.payA[q][i], pb = B.payB[q][i];
-      const float2 pc2 = B.payC[q][i];
+      float4 o = make_float4(0.0f, 0.0f, 0.0f, 0.0f), d = make_float4(0.0f, 0.0f, 1.0f, 0.0f);
+      float4 hv = make_float4(0.0f, 0.0f, 0.0f, 0.0f), pa = hv, pb = hv;
+      float2 pc2 = make_float2(0.0f, 0.0f);  // direct and indirect are zero before the first shadow ray is shaded
+      float dLight = 0.0f;
+      if (!extension) {
+        o = B.rayO[q][i];
+        d = B.rayD[q][i];
+        pa = B.payA[q][i];
+      }
+      if (generic || extension) hv = B.hits[i];
+      else hv.w = __int_as_float(wf_hit_words(B)[i]);
+      if (K != WF_FIRST_SHADOW) {
+        pb = B.payB[q][i];
+        pc2 = B.payC[q][i];
+      }
+      if (extension) dLight = wf_dlight(B, q)[i];
       r.ox = o.x; r.oy = o.y; r.oz = o.z;
       r.dx = d.x; r.dy = d.y; r.dz = d.z;
       Hit h;
@@ -437,16 +489,17 @@ __global__ void __launch_bounds__(WF_BLOCK, 8) k_wf_shade(LtSceneDev sc, LtLaunc
       h.prim = (int)(hb & 0x7fffffffu);
       h.hit = (int)(hb >> 31);
       PathState ps;
-      ps.stage = (word >> WF_PATH_BITS) & 3;
+      ps.stage = generic ? (word >> WF_PATH_BITS) & 3
+                         : (K == WF_FIRST_SHADOW ? ST_SHADOW_DIRECT : (K == WF_SHADOW ? ST_SHADOW_EXT : ST_EXTENSION));
       ps.depth = (int)((unsigned)word >> (WF_PATH_BITS + 2));
       // every ray after the primary one ignores the primitive its path stands on (basic_lighting.cl:271,
-      // global_illumination.cl:294,311,350)
+      // global_illumination.cl:294,311,350); an extension result sets it or does not read it
       ps.hitPrim = (int)((unsigned)__float_as_int(d.w) & 0x7fffffffu) - 1;
       const bool shadowStage = ps.stage == ST_SHADOW_DIRECT || ps.stage == ST_SHADOW_EXT;
       const bool lightHit = ps.stage == ST_EXTENSION && is_light(sc, h.prim);
       const bool surfaceHit = ps.stage == ST_EXTENSION && !lightHit && h.hit == 1;
       ps.nrm[0] = pa.x; ps.nrm[1] = pa.y; ps.nrm[2] = pa.z;
-      ps.extW = pa.w;  // read by the light hit of an extension ray only
+      ps.dLight = extension ? dLight : pa.w;  // read by the light hit of an extension ray only
       ps.diffuse[0] = ps.diffuse[1] = ps.diffuse[2] = 0.0f;  // an extension result sets it or does not read it
       if (shadowStage) {
         const RefMaterial* mat = sc.mats + __float_as_int(pa.w);
@@ -471,11 +524,11 @@ __global__ void __launch_bounds__(WF_BLOCK, 8) k_wf_shade(LtSceneDev sc, LtLaunc
       } else {
         emit = true;
         // a surface hit is the new shading point of a shadow ray; otherwise the next ray is an extension ray
-        pl = wf_payload(ps, surfaceHit ? __int_as_float(sc.prims[h.prim].materialIndex) : ps.extW);
+        pl = wf_payload(ps, surfaceHit ? __int_as_float(sc.prims[h.prim].materialIndex) : ps.dLight);
         path = wf_pack_path(path, ps.stage, ps.depth);
       }
     }
-    queue_append(B, 1 - q, emit, r, tStart, ignore, anyHit, path, pl, lane);
+    queue_append<OUT>(B, 1 - q, emit, r, tStart, ignore, anyHit, path, pl, lane);
   }
 }
 
@@ -514,7 +567,8 @@ __global__ void __launch_bounds__(WF_BLOCK) k_wf_accumulate(LtLaunch L, LtWfBuff
 // host side
 // ------------------------------------------------------------------------------------------------
 size_t lt_wf_bytes_per_path() {
-  // frame colour, hits; per queue: ray (2 x 16 B), payload (40 B), path word
+  // frame colour, hits; per queue: ray (2 x 16 B), payload (40 B), path word.  The hit words and dLight live inside
+  // the hits and payA arrays (wf_hit_words, wf_dlight).
   return sizeof(float4) * 2 + 2 * (sizeof(float4) * 4 + sizeof(float2) + sizeof(int));
 }
 
@@ -560,6 +614,26 @@ size_t lt_wf_primary_hits_bytes(long long pixels) {
 const void* const lt_wf_traversal_kernels[5] = {
     (const void*)k_wf_primary_trace, (const void*)k_wf_primary<false>, (const void*)k_wf_primary<true>,
     (const void*)k_wf_trace<false, false>, (const void*)k_wf_trace<true, false>};
+
+// Round r >= 1 of a sample (WfRound).  The exact pipelines fold the retracing of a light hit into its shading, so round
+// 1 holds the first shadow rays of the paths, and after it extension and shadow rounds alternate: an extension result
+// emits only shadow rays, a shadow result only extension rays.  Counting launches that retrace light hits append
+// extension rays to shadow rounds.
+static int wf_round_kind(int flags, int r) {
+  if (!lt_fold_light_hits(flags)) return WF_GENERIC;
+  return r == 1 ? WF_FIRST_SHADOW : (r & 1) ? WF_SHADOW : WF_EXTENSION;
+}
+
+template <int Q>
+static void launch_shade(int kind, int grid, cudaStream_t st, const LtSceneDev& sc, const LtLaunch& L,
+                         const LtWfBuffers& B, int pixels, int sample, const LtWfPrimary& P) {
+  switch (kind) {
+    case WF_FIRST_SHADOW: k_wf_shade<Q, WF_FIRST_SHADOW><<<grid, WF_BLOCK, 0, st>>>(sc, L, B, pixels, 0, sample, P); break;
+    case WF_SHADOW: k_wf_shade<Q, WF_SHADOW><<<grid, WF_BLOCK, 0, st>>>(sc, L, B, pixels, 0, sample, P); break;
+    case WF_EXTENSION: k_wf_shade<Q, WF_EXTENSION><<<grid, WF_BLOCK, 0, st>>>(sc, L, B, pixels, 0, sample, P); break;
+    default: k_wf_shade<Q, WF_GENERIC><<<grid, WF_BLOCK, 0, st>>>(sc, L, B, pixels, 0, sample, P); break;
+  }
+}
 
 int lt_launch_render_wavefront(const LtSceneDev& sc, const LtPlan& plan, const LtLaunch& L, float* dOut,
                                LtCounters* dCounters, void* workspace, int smCount, cudaStream_t stream,
@@ -632,20 +706,23 @@ int lt_launch_render_wavefront(const LtSceneDev& sc, const LtPlan& plan, const L
       k_wf_reset<<<1, 1, 0, st>>>(B);
       // a traversal kernel only when it traces the camera rays itself
       mark(0, st, primaryHits ? LT_TIMED_PRIMARY_SHADE : LT_TIMED_TRAVERSAL);
-      if (stats) k_wf_primary<true><<<grid, WF_BLOCK, smem, st>>>(sc, Lb, B, nf, pixels, s, dCounters, P);
-      else k_wf_primary<false><<<grid, WF_BLOCK, smem, st>>>(sc, Lb, B, nf, pixels, s, nullptr, P);
+      const int out = wf_round_kind(L.flags, 1);
+      if (stats) k_wf_primary<true><<<grid, WF_BLOCK, smem, st>>>(sc, Lb, B, nf, pixels, s, dCounters, P, out);
+      else k_wf_primary<false><<<grid, WF_BLOCK, smem, st>>>(sc, Lb, B, nf, pixels, s, nullptr, P, out);
       mark(1, st, primaryHits ? LT_TIMED_PRIMARY_SHADE : LT_TIMED_TRAVERSAL);
       launches += 2;
       int q = 0;
       for (int r = 1; r < plan.rounds; r++) {
+        const int kind = wf_round_kind(L.flags, r);
+        int* hitWords = (kind == WF_FIRST_SHADOW || kind == WF_SHADOW) ? (int*)B.hits : nullptr;  // wf_hit_words
         mark(0, st);
-        if (stats) k_wf_trace<true, false><<<plan.grid, WF_BLOCK, smem, st>>>(sc, Lb, B, q, dCounters, B.rayO[q], B.rayD[q]);
-        else if (threaded) k_wf_trace<false, true><<<plan.grid, WF_BLOCK, plan.smemTrace, st>>>(sc, Lb, B, q, nullptr, B.rayO[q], B.rayD[q]);
-        else k_wf_trace<false, false><<<plan.grid, WF_BLOCK, smem, st>>>(sc, Lb, B, q, nullptr, B.rayO[q], B.rayD[q]);
+        if (stats) k_wf_trace<true, false><<<plan.grid, WF_BLOCK, smem, st>>>(sc, Lb, B, q, dCounters, B.rayO[q], B.rayD[q], hitWords);
+        else if (threaded) k_wf_trace<false, true><<<plan.grid, WF_BLOCK, plan.smemTrace, st>>>(sc, Lb, B, q, nullptr, B.rayO[q], B.rayD[q], hitWords);
+        else k_wf_trace<false, false><<<plan.grid, WF_BLOCK, smem, st>>>(sc, Lb, B, q, nullptr, B.rayO[q], B.rayD[q], hitWords);
         mark(1, st);
         mark(0, st, LT_TIMED_SHADE);
-        if (q == 0) k_wf_shade<0><<<grid, WF_BLOCK, 0, st>>>(sc, Lb, B, pixels, 0, s, P);
-        else k_wf_shade<1><<<grid, WF_BLOCK, 0, st>>>(sc, Lb, B, pixels, 0, s, P);
+        if (q == 0) launch_shade<0>(kind, grid, st, sc, Lb, B, pixels, s, P);
+        else launch_shade<1>(kind, grid, st, sc, Lb, B, pixels, s, P);
         mark(1, st, LT_TIMED_SHADE);
         k_wf_swap<<<1, 1, 0, st>>>(B, q);
         launches += 3;
