@@ -117,14 +117,11 @@ struct LtSceneDev {
   int stackDepth;             // entries a traversal stack needs (tree depth), <= 64
   int nodeCount, primCount, matCount;
   int prunedBase, prunedStride;  // pruned copy o of tnodes: records [prunedBase + o * prunedStride, + prunedStride);
-                                 // 0 and nodeCount: the full copies (tnodesCoherent, or no pruned copies)
+                                 // 0 and nodeCount: the full copies (device-built copies, or no pruned copies)
   const LtThreadNode* tnodes;  // 8 * nodeCount full threaded records, then the pruned ones, or NULL (scene too large)
   const int* rank;  // [8][primCount]: position, in octant o's reference visit order, of the leaf whose primitive is p;
                     // set when the pruned copies are a traversal tree (NULL otherwise).  The reference keeps the first
                     // of several triangles with equal t, i.e. the least (t, rank): tri_test breaks equal-t ties by it
-  const LtThreadNode* tnodesCoherent;  // the same records for a large scene (built on the device), used only by the
-                                       // lighting kernels' megakernel launches (camera rays + shadow rays towards a
-                                       // light): incoherent rays spread over eight copies that no longer fit in L2
 };
 
 
@@ -143,6 +140,7 @@ struct LtSceneDev {
 __constant__ LtSceneDev lt_scene;  // set by the library before each launch of a plug-in that references it
 
 #define LT_THREAD_STRIDE (blockDim.x * blockDim.y * blockDim.z)  // plug-ins run any block shape
+#define LT_THREAD_INDEX ((threadIdx.z * blockDim.y + threadIdx.y) * blockDim.x + threadIdx.x)
 #include "lt_device.cuh"
 
 struct LtRay {
@@ -168,16 +166,12 @@ struct LtHit {
 // triangle (valid when only hitType is read, as the reference's shadow rays do).
 __device__ __forceinline__ LtHit lt_trace(const LtRay& r, float tMax, int ignorePrimitiveIndex = -1, bool anyHit = false,
                                           float epsilon = LT_EPSILON_BASIC) {
-  extern __shared__ int lt_plugin_smem[];
-  const unsigned threads = blockDim.x * blockDim.y * blockDim.z;
-  const unsigned tid = (threadIdx.z * blockDim.y + threadIdx.y) * blockDim.x + threadIdx.x;
-  int* stk = lt_plugin_smem + tid;
-  int* list = lt_plugin_smem + (lt_scene.tnodes ? 0 : lt_stack_levels(lt_scene)) * threads + tid;
+  LT_TRAV_SMEM(s, lt_scene.tnodes ? 0 : lt_stack_levels(lt_scene))
   Trav t;
   t.r.ox = r.ox; t.r.oy = r.oy; t.r.oz = r.oz;
   t.r.dx = r.dx; t.r.dy = r.dy; t.r.dz = r.dz;
   LtCounters cnt = {0, 0, 0};
-  trace<false>(t, lt_scene, ignorePrimitiveIndex, tMax, epsilon, anyHit, stk, list, cnt);
+  trace<false>(t, lt_scene, ignorePrimitiveIndex, tMax, epsilon, anyHit, s, cnt);
   LtHit h;
   h.t = t.h.t; h.u = t.h.u; h.v = t.h.v;
   h.primitiveIndex = t.h.prim;

@@ -139,10 +139,6 @@ static LtTree lt_plan_threaded_copies(int nNodes, size_t totalMem, const LtLimit
   return LT_TREE_CHILD_PAIR;
 }
 
-static size_t stack_smem(int stackDepth, bool cull) {  // the layout of LT_SMEM_POINTERS (lt_device.cuh)
-  return (size_t)((stackDepth < 1 ? 1 : stackDepth) * (cull ? 2 : 1) + LT_MAX_BATCH) * LT_BLOCK * sizeof(int);
-}
-
 // The threaded copies serve the exact, uncounted kernels only: the stats kernels count in the stack traversal, whose
 // tests are the same ones, the culled traversal has no threaded form, and LT_FLAG_NO_THREADED selects the stack
 // traversal for comparison.  A large scene's device-built copies serve coherent launches only (camera rays and shadow
@@ -163,7 +159,7 @@ static LtPlan lt_plan_primary_hits(int flags, int width, int height, const LtSce
   p.pipeline = LT_PIPE_FLAT;
   p.tree = plan_tree(flags, false, s.copies);
   p.cull = (flags & LT_FLAG_CULL) != 0;
-  p.smemStack = p.smemTrace = stack_smem(s.stackDepth, p.cull);
+  p.smemStack = p.smemTrace = lt_traversal_smem(lt_stack_levels(s), LT_BLOCK, p.cull);
   p.grid = tile_blocks(width, height);
   return p;
 }
@@ -232,8 +228,8 @@ static LtPlan lt_plan_render(const LtLaunch& L, const LtSceneFacts& s, size_t to
   const bool coherent =
       p.pipeline == LT_PIPE_PATH && (L.kernel == LT_KERNEL_LIGHTING25 || L.kernel == LT_KERNEL_ACCUMULATOR);
   p.tree = plan_tree(L.flags, coherent, s.copies);
-  p.smemStack = stack_smem(s.stackDepth, p.cull);
-  p.smemTrace = p.tree == LT_TREE_CHILD_PAIR ? p.smemStack : (size_t)LT_MAX_BATCH * LT_BLOCK * sizeof(int);
+  p.smemStack = lt_traversal_smem(lt_stack_levels(s), LT_BLOCK, p.cull);
+  p.smemTrace = p.tree == LT_TREE_CHILD_PAIR ? p.smemStack : lt_traversal_smem(0, LT_BLOCK, false);
   // shared memory is what limits residency of the persistent kernels (the threaded trace kernel's 8 KB: the cap of
   // 8); k_flat_stream measured at 4 .. 10: no difference (the longest tile bounds the kernel)
   p.blocksPerSm = (int)((200 * 1024) / p.smemTrace);
@@ -810,7 +806,6 @@ static int finish_scene(lt_ctx* ctx, lt_scene* s, int nNodes, int nPrims, int nM
   d.matCount = nMats;
   d.tnodes = s->dThread;
   d.rank = s->dRank;
-  d.tnodesCoherent = s->dThreadBig;
   set_pruned_copies(s, false);
   return LT_OK;
 }

@@ -14,10 +14,11 @@
 #endif
 
 // Per-thread stacks and leaf FIFOs live in shared memory as [level][thread]: LT_THREAD_STRIDE ints between the levels
-// of one thread.  The library's kernels run blocks of LT_BLOCK threads; a plug-in build (any block shape) defines
-// the stride as its run-time block size before including this file.
+// of one thread, LT_THREAD_INDEX the thread's column.  The library's kernels run blocks of LT_BLOCK threads; a plug-in
+// build (any block shape) defines both from its run-time block shape before including this file.
 #ifndef LT_THREAD_STRIDE
 #define LT_THREAD_STRIDE LT_BLOCK
+#define LT_THREAD_INDEX threadIdx.x
 #endif
 #define LT_LEVEL_BYTES ((unsigned)(LT_THREAD_STRIDE) * 4u)
 
@@ -142,29 +143,41 @@ __device__ __forceinline__ bool finite3(float a, float b, float c) {
   return fabsf(a) <= FLT_MAX && fabsf(b) <= FLT_MAX && fabsf(c) <= FLT_MAX;
 }
 
+// the select-chain test of the box (min, max) per axis, with lo/hi chosen by the ray's sign mask (basic.cu:88-91)
+__device__ __forceinline__ bool slab_exact(const Trav& t, float mnx, float mxx, float mny, float mxy, float mnz,
+                                           float mxz) {
+  bool nx = t.negMask & 1u, ny = t.negMask & 2u, nz = t.negMask & 4u;
+  return slab(nx ? mxx : mnx, nx ? mnx : mxx, ny ? mxy : mny, ny ? mny : mxy, nz ? mxz : mnz, nz ? mnz : mxz, t.r,
+              t.ix, t.iy, t.iz);
+}
+
 __device__ __forceinline__ bool box_test(const Trav& t, float mnx, float mxx, float mny, float mxy, float mnz,
                                          float mxz) {
-  if (t.negMask & LT_EXACT_SLAB) {
-    bool nx = t.negMask & 1u, ny = t.negMask & 2u, nz = t.negMask & 4u;
-    return slab(nx ? mxx : mnx, nx ? mnx : mxx, ny ? mxy : mny, ny ? mny : mxy, nz ? mxz : mnz, nz ? mnz : mxz, t.r,
-                t.ix, t.iy, t.iz);
-  }
+  if (t.negMask & LT_EXACT_SLAB) return slab_exact(t, mnx, mxx, mny, mxy, mnz, mxz);
   return slab_fast(mnx, mxx, mny, mxy, mnz, mxz, t.r, t.ix, t.iy, t.iz);
+}
+
+// the part of starting a ray that every walk shares: reciprocals, sign mask, empty hit record, stack and leaf FIFO.
+// Returns the ray's sign octant (negMask without LT_EXACT_SLAB).
+__device__ __forceinline__ int trav_setup(Trav& t, int ignore, float tInit, bool anyHit) {
+  t.ix = FRCP(t.r.dx);
+  t.iy = FRCP(t.r.dy);
+  t.iz = FRCP(t.r.dz);
+  t.negMask = (t.ix < 0.0f ? 1u : 0u) | (t.iy < 0.0f ? 2u : 0u) | (t.iz < 0.0f ? 4u : 0u);
+  const int oct = (int)t.negMask;
+  if (!(finite3(t.ix, t.iy, t.iz) && finite3(t.r.ox, t.r.oy, t.r.oz))) t.negMask |= LT_EXACT_SLAB;
+  t.h.t = tInit; t.h.u = 0.0f; t.h.v = 0.0f; t.h.prim = 0; t.h.hit = 0;
+  t.ignore = ignore;
+  t.anyHit = anyHit;
+  t.sp = 0;
+  t.qHead = t.qTail = 0;
+  return oct;
 }
 
 template <bool STATS>
 __device__ __forceinline__ void trav_begin(Trav& t, const LtSceneDev& sc, int ignore, float tInit, bool anyHit,
                                            LtCounters& cnt) {
-  t.ix = FRCP(t.r.dx);
-  t.iy = FRCP(t.r.dy);
-  t.iz = FRCP(t.r.dz);
-  t.negMask = (t.ix < 0.0f ? 1u : 0u) | (t.iy < 0.0f ? 2u : 0u) | (t.iz < 0.0f ? 4u : 0u);
-  if (!(finite3(t.ix, t.iy, t.iz) && finite3(t.r.ox, t.r.oy, t.r.oz))) t.negMask |= LT_EXACT_SLAB;
-  t.h.t = tInit; t.h.u = 0.0f; t.h.v = 0.0f; t.h.prim = 0; t.h.hit = 0;
-  t.ignore = ignore;
-  t.anyHit = STATS ? false : anyHit;
-  t.sp = 0;
-  t.qHead = t.qTail = 0;
+  trav_setup(t, ignore, tInit, STATS ? false : anyHit);
   if (STATS) {
     cnt.rays++;
     cnt.nodeTests++;
@@ -208,9 +221,14 @@ __device__ __forceinline__ void ldg256(const void* p, float4& a, float4& b) {
 #endif
 }
 
-// one inner-node step; requires t.cur >= 0
+// the two child boxes of inner node t.cur, in the order the reference visits them
+struct NodePair {
+  int nearRef, farRef;
+  bool hn, hf;  // near / far child box hit
+};
+
 template <bool STATS>
-__device__ __forceinline__ void trav_node_step(Trav& t, const LtSceneDev& sc, int* __restrict__ stk, LtCounters& cnt) {
+__device__ __forceinline__ NodePair node_pair_test(const Trav& t, const LtSceneDev& sc, LtCounters& cnt) {
   const float4* np = reinterpret_cast<const float4*>(sc.wnodes + t.cur);
   float4 bx, by, bz, mf;
   ldg256(np, bx, by);
@@ -221,11 +239,8 @@ __device__ __forceinline__ void trav_node_step(Trav& t, const LtSceneDev& sc, in
   // non-finite reciprocals; both give the same answer where both apply.  If any lane that is at this
   // instruction needs the select chain, all of them take it: one instruction stream per warp.
   if (__any_sync(__activemask(), (t.negMask & LT_EXACT_SLAB) != 0u)) {
-    bool nx = t.negMask & 1u, ny = t.negMask & 2u, nz = t.negMask & 4u;
-    hl = slab(nx ? bx.y : bx.x, nx ? bx.x : bx.y, ny ? by.y : by.x, ny ? by.x : by.y, nz ? bz.y : bz.x,
-              nz ? bz.x : bz.y, t.r, t.ix, t.iy, t.iz);
-    hr = slab(nx ? bx.w : bx.z, nx ? bx.z : bx.w, ny ? by.w : by.z, ny ? by.z : by.w, nz ? bz.w : bz.z,
-              nz ? bz.z : bz.w, t.r, t.ix, t.iy, t.iz);
+    hl = slab_exact(t, bx.x, bx.y, by.x, by.y, bz.x, bz.y);
+    hr = slab_exact(t, bx.z, bx.w, by.z, by.w, bz.z, bz.w);
   } else {
     hl = slab_fast(bx.x, bx.y, by.x, by.y, bz.x, bz.y, t.r, t.ix, t.iy, t.iz);
     hr = slab_fast(bx.z, bx.w, by.z, by.w, bz.z, bz.w, t.r, t.ix, t.iy, t.iz);
@@ -240,16 +255,26 @@ __device__ __forceinline__ void trav_node_step(Trav& t, const LtSceneDev& sc, in
   // near child first by the sign of the direction on the split axis (basic.cu:180-186); written
   // with selects so the lanes of a warp do not split on the four hit/miss combinations
   bool axisNeg = (t.negMask >> m.z) & 1u;
-  int nearRef = axisNeg ? m.y : m.x, farRef = axisNeg ? m.x : m.y;
-  bool hn = axisNeg ? hr : hl, hf = axisNeg ? hl : hr;
-  bool both = hn && hf, none = !hn && !hf;
+  NodePair p;
+  p.nearRef = axisNeg ? m.y : m.x;
+  p.farRef = axisNeg ? m.x : m.y;
+  p.hn = axisNeg ? hr : hl;
+  p.hf = axisNeg ? hl : hr;
+  return p;
+}
+
+// one inner-node step; requires t.cur >= 0
+template <bool STATS>
+__device__ __forceinline__ void trav_node_step(Trav& t, const LtSceneDev& sc, int* __restrict__ stk, LtCounters& cnt) {
+  const NodePair p = node_pair_test<STATS>(t, sc, cnt);
+  bool both = p.hn && p.hf, none = !p.hn && !p.hf;
   bool canPop = none && t.sp > 0;
   t.sp -= canPop ? 1 : 0;
   int slot = t.sp * LT_THREAD_STRIDE;
   int popped = stk[slot];
-  if (both) stk[slot] = farRef;
+  if (both) stk[slot] = p.farRef;
   t.sp += both ? 1 : 0;
-  t.cur = hn ? nearRef : (hf ? farRef : (canPop ? popped : LT_DONE));
+  t.cur = p.hn ? p.nearRef : (p.hf ? p.farRef : (canPop ? popped : LT_DONE));
 }
 
 // Traversal never depends on triangle results (the reference does not cull by t, basic.cu:136-154),
@@ -280,6 +305,13 @@ __device__ __forceinline__ int trav_collect(Trav& t, const LtSceneDev& sc, int* 
   return n;
 }
 
+// triangle `prim` replaced the hit record (tri_test): record it.  Returns true when that finishes the ray (any hit).
+__device__ __forceinline__ bool accept_hit(Trav& t, int prim) {
+  t.h.prim = prim;
+  t.h.hit = 1;
+  return t.anyHit;
+}
+
 // leaf phase: test the recorded triangles in order.  Returns true if the ray is finished early
 // (any-hit ray that found a hit).
 template <bool STATS>
@@ -288,16 +320,42 @@ __device__ __forceinline__ bool trav_test(Trav& t, const LtSceneDev& sc, const i
   for (int i = 0; i < n; i++) {
     int prim = list[i * LT_THREAD_STRIDE];
     if (STATS) cnt.triTests++;
-    if (tri_test(sc.tris, prim, t.r, epsThr, t.h, nullptr)) {
-      t.h.prim = prim;
-      t.h.hit = 1;
-      if (t.anyHit) {
-        t.cur = LT_DONE;
-        return true;
-      }
+    if (tri_test(sc.tris, prim, t.r, epsThr, t.h, nullptr) && accept_hit(t, prim)) {
+      t.cur = LT_DONE;
+      return true;
     }
   }
   return false;
+}
+
+// ---- leaf FIFO of the pipelined and threaded walks: LT_MAX_BATCH entries per thread in shared memory, ------------
+// addressed through 32-bit shared addresses; t.qHead / t.qTail count pops and pushes
+__device__ __forceinline__ unsigned fifo_addr(unsigned fifoAddr, int q) {
+  return fifoAddr + ((unsigned)(q & (LT_MAX_BATCH - 1)) * LT_LEVEL_BYTES);
+}
+__device__ __forceinline__ void fifo_push(Trav& t, unsigned fifoAddr, int prim) {
+  sts32(fifo_addr(fifoAddr, t.qTail), prim);
+  t.qTail++;
+}
+__device__ __forceinline__ int fifo_pop(Trav& t, unsigned fifoAddr) {
+  int prim = lds32(fifo_addr(fifoAddr, t.qHead));
+  t.qHead++;
+  return prim;
+}
+
+// test up to n recorded triangles, oldest first (tri_test's rank / row); an any-hit ray that hits empties the FIFO
+// and is finished
+template <bool STATS>
+__device__ __forceinline__ void fifo_drain(Trav& t, const LtSceneDev& sc, unsigned fifoAddr, float epsThr, int n,
+                                           const int* __restrict__ rank, int row, LtCounters& cnt) {
+  for (int k = 0; k < n && t.qHead != t.qTail; k++) {
+    int prim = fifo_pop(t, fifoAddr);
+    if (STATS) cnt.triTests++;
+    if (tri_test(sc.tris, prim, t.r, epsThr, t.h, rank, row) && accept_hit(t, prim)) {
+      t.cur = LT_DONE;
+      t.qHead = t.qTail;
+    }
+  }
 }
 
 // ---- software-pipelined traversal for the persistent loops (k_flat_stream, k_wf_trace) ----------
@@ -318,83 +376,35 @@ __device__ __forceinline__ bool trav_iter_lean(Trav& t, const LtSceneDev& sc, un
   // one step records up to three leaves (near child, far child, and a leaf popped behind them)
   for (int steps = 0; steps < nodeSteps && t.cur != LT_DONE && t.qTail - t.qHead <= LT_MAX_BATCH - 3; steps++) {
     if (t.cur >= 0) {
-      const float4* np = reinterpret_cast<const float4*>(sc.wnodes + t.cur);
-      float4 bx, by, bz, mf;
-      ldg256(np, bx, by);
-      ldg256(np + 2, bz, mf);
-      int4 m = make_int4(__float_as_int(mf.x), __float_as_int(mf.y), __float_as_int(mf.z), __float_as_int(mf.w));
-      unsigned hits;  // bit 0: left child box hit, bit 1: right child box hit
-      if (__any_sync(__activemask(), (t.negMask & LT_EXACT_SLAB) != 0u)) {
-        bool nx = t.negMask & 1u, ny = t.negMask & 2u, nz = t.negMask & 4u;
-        bool hl = slab(nx ? bx.y : bx.x, nx ? bx.x : bx.y, ny ? by.y : by.x, ny ? by.x : by.y, nz ? bz.y : bz.x,
-                       nz ? bz.x : bz.y, t.r, t.ix, t.iy, t.iz);
-        bool hr = slab(nx ? bx.w : bx.z, nx ? bx.z : bx.w, ny ? by.w : by.z, ny ? by.z : by.w, nz ? bz.w : bz.z,
-                       nz ? bz.z : bz.w, t.r, t.ix, t.iy, t.iz);
-        hits = (hl ? 1u : 0u) | (hr ? 2u : 0u);
-      } else {
-        bool hl = slab_fast(bx.x, bx.y, by.x, by.y, bz.x, bz.y, t.r, t.ix, t.iy, t.iz);
-        bool hr = slab_fast(bx.z, bx.w, by.z, by.w, bz.z, bz.w, t.r, t.ix, t.iy, t.iz);
-        hits = (hl ? 1u : 0u) | (hr ? 2u : 0u);
-      }
-      if (STATS) {
-        cnt.nodeTests += 2;
-        unsigned lc = (unsigned)m.w & 0xffffu, rc = (unsigned)m.w >> 16;
-        if ((hits & 1u) && m.x < 0 && lc > 1 && ~m.x != t.ignore) cnt.triTests += lc - 1;
-        if ((hits & 2u) && m.y < 0 && rc > 1 && ~m.y != t.ignore) cnt.triTests += rc - 1;
-      }
-      // near child first by the sign of the direction on the split axis (basic.cu:180-186)
-      bool axisNeg = (t.negMask >> m.z) & 1u;
-      int nearRef = axisNeg ? m.y : m.x, farRef = axisNeg ? m.x : m.y;
-      bool hn = (hits & (axisNeg ? 2u : 1u)) != 0u, hf = (hits & (axisNeg ? 1u : 2u)) != 0u;
-      bool nearInner = hn && nearRef >= 0;       // descend into near; far (if hit) must wait on the stack
-      bool recNear = hn && nearRef < 0 && ~nearRef != t.ignore;
-      bool farNow = hf && !nearInner;            // far is next in order right away
-      bool recFar = farNow && farRef < 0 && ~farRef != t.ignore;
-      if (recNear) {
-        sts32(fifoAddr + ((unsigned)(t.qTail & (LT_MAX_BATCH - 1)) * LT_LEVEL_BYTES), ~nearRef);
-        t.qTail++;
-      }
-      if (recFar) {
-        sts32(fifoAddr + ((unsigned)(t.qTail & (LT_MAX_BATCH - 1)) * LT_LEVEL_BYTES), ~farRef);
-        t.qTail++;
-      }
-      bool push = hf && nearInner;
-      bool farInner = farNow && farRef >= 0;
+      const NodePair p = node_pair_test<STATS>(t, sc, cnt);
+      bool nearInner = p.hn && p.nearRef >= 0;   // descend into near; far (if hit) must wait on the stack
+      bool recNear = p.hn && p.nearRef < 0 && ~p.nearRef != t.ignore;
+      bool farNow = p.hf && !nearInner;          // far is next in order right away
+      bool recFar = farNow && p.farRef < 0 && ~p.farRef != t.ignore;
+      if (recNear) fifo_push(t, fifoAddr, ~p.nearRef);
+      if (recFar) fifo_push(t, fifoAddr, ~p.farRef);
+      bool push = p.hf && nearInner;
+      bool farInner = farNow && p.farRef >= 0;
       bool pop = !nearInner && !farInner;
       bool canPop = pop && t.sp > 0;
       t.sp -= canPop ? 1 : 0;
       unsigned slot = stkAddr + ((unsigned)t.sp * LT_LEVEL_BYTES);
       int popped = lds32(slot);
-      if (push) sts32(slot, farRef);
+      if (push) sts32(slot, p.farRef);
       t.sp += push ? 1 : 0;
-      t.cur = nearInner ? nearRef : (farInner ? farRef : (canPop ? popped : LT_DONE));
+      t.cur = nearInner ? p.nearRef : (farInner ? p.farRef : (canPop ? popped : LT_DONE));
     }
     // a leaf that waited on the stack (or the root itself): record it and take the next entry
     if (t.cur < 0 && t.cur != LT_DONE) {
       int prim = ~t.cur;
-      if (prim != t.ignore) {
-        sts32(fifoAddr + ((unsigned)(t.qTail & (LT_MAX_BATCH - 1)) * LT_LEVEL_BYTES), prim);
-        t.qTail++;
-      }
+      if (prim != t.ignore) fifo_push(t, fifoAddr, prim);
       bool can = t.sp > 0;
       t.sp -= can ? 1 : 0;
       int v = lds32(stkAddr + ((unsigned)t.sp * LT_LEVEL_BYTES));
       t.cur = can ? v : LT_DONE;
     }
   }
-  for (int k = 0; k < triTests && t.qHead != t.qTail; k++) {
-    int prim = lds32(fifoAddr + ((unsigned)(t.qHead & (LT_MAX_BATCH - 1)) * LT_LEVEL_BYTES));
-    t.qHead++;
-    if (STATS) cnt.triTests++;
-    if (tri_test(sc.tris, prim, t.r, epsThr, t.h, nullptr)) {
-      t.h.prim = prim;
-      t.h.hit = 1;
-      if (t.anyHit) {
-        t.cur = LT_DONE;
-        t.qHead = t.qTail;
-      }
-    }
-  }
+  fifo_drain<STATS>(t, sc, fifoAddr, epsThr, triTests, nullptr, 0, cnt);
   return t.cur == LT_DONE && t.qHead == t.qTail;
 }
 
@@ -407,12 +417,7 @@ __device__ __forceinline__ bool trav_iter_lean(Trav& t, const LtSceneDev& sc, un
 // (lo - o) * inv <= (hi - o) * inv per axis and the select chain of basic.cu:136-154 reduces to
 // max3(entries) <= min3(exits) && min3(exits) > 0 on the same FSUB/FMUL products.
 __device__ __forceinline__ void trav_begin_threaded(Trav& t, const LtSceneDev& sc, int ignore, float tInit, bool anyHit) {
-  t.ix = FRCP(t.r.dx);
-  t.iy = FRCP(t.r.dy);
-  t.iz = FRCP(t.r.dz);
-  t.negMask = (t.ix < 0.0f ? 1u : 0u) | (t.iy < 0.0f ? 2u : 0u) | (t.iz < 0.0f ? 4u : 0u);
-  const int oct = (int)(t.negMask & 7u);
-  if (!(finite3(t.ix, t.iy, t.iz) && finite3(t.r.ox, t.r.oy, t.r.oz))) t.negMask |= LT_EXACT_SLAB;
+  const int oct = trav_setup(t, ignore, tInit, anyHit);
   // the pruned copies rely on (b - o) * inv being monotonic in the bound b: not so for a non-finite reciprocal or
   // origin, nor for a zero reciprocal (inf * 0 = NaN when b - o overflows); those rays walk the full copies
   const bool full = (t.negMask & LT_EXACT_SLAB) || t.ix == 0.0f || t.iy == 0.0f || t.iz == 0.0f;
@@ -423,11 +428,6 @@ __device__ __forceinline__ void trav_begin_threaded(Trav& t, const LtSceneDev& s
   if (sc.rootRef >= 0)
     t.cur = box_test(t, sc.rootMin[0], sc.rootMax[0], sc.rootMin[1], sc.rootMax[1], sc.rootMin[2], sc.rootMax[2])
                 ? rootRecord + 1 : LT_DONE;
-  t.h.t = tInit; t.h.u = 0.0f; t.h.v = 0.0f; t.h.prim = 0; t.h.hit = 0;
-  t.ignore = ignore;
-  t.anyHit = anyHit;
-  t.sp = 0;
-  t.qHead = t.qTail = 0;
 }
 
 // node phase, EXACT = select chain (valid for every ray) or interval form (rays with finite reciprocals).
@@ -455,10 +455,7 @@ __device__ __forceinline__ void trav_threaded_nodes(Trav& t, const LtThreadNode*
       hit = lo <= hi && hi > 0.0f;
     }
     int link = __float_as_int(b.z), skip = __float_as_int(b.w);
-    if (hit && link < 0 && link != notIgnore) {
-      sts32(fifoAddr + ((unsigned)(t.qTail & (LT_MAX_BATCH - 1)) * LT_LEVEL_BYTES), ~link);
-      t.qTail++;
-    }
+    if (hit && link < 0 && link != notIgnore) fifo_push(t, fifoAddr, ~link);
     t.cur = (hit && link >= 0) ? t.cur + 1 : skip;
   }
 }
@@ -475,18 +472,8 @@ __device__ __forceinline__ bool trav_iter_threaded(Trav& t, const LtSceneDev& sc
   const int notIgnore = ~t.ignore;  // a leaf's link is ~primitivesOffset
   if (exact) trav_threaded_nodes<true>(t, sc.tnodes, fifoAddr, maxSteps, notIgnore);
   else trav_threaded_nodes<false>(t, sc.tnodes, fifoAddr, maxSteps, notIgnore);
-  for (int k = 0; k < triTests && t.qHead != t.qTail; k++) {
-    int prim = lds32(fifoAddr + ((unsigned)(t.qHead & (LT_MAX_BATCH - 1)) * LT_LEVEL_BYTES));
-    t.qHead++;
-    if (tri_test(sc.tris, prim, t.r, epsThr, t.h, sc.rank, (int)(t.negMask & 7u) * sc.primCount)) {
-      t.h.prim = prim;
-      t.h.hit = 1;
-      if (t.anyHit) {
-        t.cur = LT_DONE;
-        t.qHead = t.qTail;
-      }
-    }
-  }
+  LtCounters uncounted = {0, 0, 0};  // counting launches take the stack traversal
+  fifo_drain<false>(t, sc, fifoAddr, epsThr, triTests, sc.rank, (int)(t.negMask & 7u) * sc.primCount, uncounted);
   return t.cur == LT_DONE && t.qHead == t.qTail;
 }
 
@@ -526,11 +513,8 @@ __device__ __forceinline__ void trav_step_cull(Trav& t, const LtSceneDev& sc, in
     bool hl, hr;
     float el = -FLT_MAX, er = -FLT_MAX;
     if (t.negMask & LT_EXACT_SLAB) {
-      bool nx = t.negMask & 1u, ny = t.negMask & 2u, nz = t.negMask & 4u;
-      hl = slab(nx ? bx.y : bx.x, nx ? bx.x : bx.y, ny ? by.y : by.x, ny ? by.x : by.y, nz ? bz.y : bz.x,
-                nz ? bz.x : bz.y, t.r, t.ix, t.iy, t.iz);
-      hr = slab(nx ? bx.w : bx.z, nx ? bx.z : bx.w, ny ? by.w : by.z, ny ? by.z : by.w, nz ? bz.w : bz.z,
-                nz ? bz.z : bz.w, t.r, t.ix, t.iy, t.iz);
+      hl = slab_exact(t, bx.x, bx.y, by.x, by.y, bz.x, bz.y);
+      hr = slab_exact(t, bx.z, bx.w, by.z, by.w, bz.z, bz.w);
     } else {
       hl = slab_fast_entry(bx.x, bx.y, by.x, by.y, bz.x, bz.y, t.r, t.ix, t.iy, t.iz, el);
       hr = slab_fast_entry(bx.z, bx.w, by.z, by.w, bz.z, bz.w, t.r, t.ix, t.iy, t.iz, er);
@@ -560,10 +544,7 @@ __device__ __forceinline__ void trav_step_cull(Trav& t, const LtSceneDev& sc, in
     int prim = ~t.cur;
     if (prim != t.ignore) {
       if (STATS) cnt.triTests++;
-      if (tri_test(sc.tris, prim, t.r, epsThr, t.h, nullptr)) {
-        t.h.prim = prim;
-        t.h.hit = 1;
-      }
+      if (tri_test(sc.tris, prim, t.r, epsThr, t.h, nullptr)) accept_hit(t, prim);  // closest hit: never finishes
     }
   }
   // pop the next stacked reference whose box entry is still within the limit
@@ -578,37 +559,51 @@ __device__ __forceinline__ void trav_step_cull(Trav& t, const LtSceneDev& sc, in
   }
 }
 
+// This thread's part of a traversal's dynamic shared memory (layout: lt_traversal_smem, lt_device_types.h) when
+// `levels` stack levels are reserved: stack, leaf list / FIFO (also as 32-bit shared addresses) and entry distances.
+struct TravSmem {
+  int* stk;
+  int* list;
+  float* tstk;  // culled launches only
+  unsigned stkAddr, fifoAddr;
+};
+
+// Declares `TravSmem s` in a kernel.  A macro rather than a function returning the struct: written out in the kernel
+// body, ptxas schedules k_path, k_flat and k_primary_hits exactly as with separate pointers (a returned struct changed
+// k_path's schedule and cost it 3 % on B200).
+#define LT_TRAV_SMEM(s, levels)                                                                                \
+  TravSmem s;                                                                                                  \
+  {                                                                                                            \
+    extern __shared__ int lt_traversal_shared[];                                                               \
+    s.stk = lt_traversal_shared + LT_THREAD_INDEX;                                                             \
+    s.list = lt_traversal_shared + (levels) * LT_THREAD_STRIDE + LT_THREAD_INDEX;                              \
+    s.tstk = reinterpret_cast<float*>(lt_traversal_shared + ((levels) + LT_MAX_BATCH) * LT_THREAD_STRIDE) +    \
+             LT_THREAD_INDEX;                                                                                  \
+    s.stkAddr = (unsigned)__cvta_generic_to_shared(s.stk);                                                     \
+    s.fifoAddr = (unsigned)__cvta_generic_to_shared(s.list);                                                   \
+  }
+
 template <bool STATS>
 __device__ __forceinline__ void trace_cull(Trav& t, const LtSceneDev& sc, int ignore, float tInit, float epsThr,
-                                           int* __restrict__ stk, float* __restrict__ tstk, LtCounters& cnt) {
+                                           const TravSmem& s, LtCounters& cnt) {
   trav_begin<STATS>(t, sc, ignore, tInit, false, cnt);
-  while (t.cur != LT_DONE) trav_step_cull<STATS>(t, sc, stk, tstk, epsThr, cnt);
+  while (t.cur != LT_DONE) trav_step_cull<STATS>(t, sc, s.stk, s.tstk, epsThr, cnt);
 }
-
-// dynamic shared memory of every traversal kernel: [stackDepth][LT_BLOCK] stack, [LT_MAX_BATCH][LT_BLOCK] leaf
-// list/FIFO, [stackDepth][LT_BLOCK] entry distances (culled mode only); lt_capi.cu: stack_smem sizes it
-__host__ __device__ inline int lt_stack_levels(const LtSceneDev& sc) { return sc.stackDepth < 1 ? 1 : sc.stackDepth; }
-#define LT_SMEM_POINTERS(sc)                                                            \
-  extern __shared__ int smemStack[];                                                    \
-  int* stk = smemStack + threadIdx.x;                                                   \
-  int* list = smemStack + lt_stack_levels(sc) * LT_BLOCK + threadIdx.x;                 \
-  float* tstk = reinterpret_cast<float*>(smemStack + (lt_stack_levels(sc) + LT_MAX_BATCH) * LT_BLOCK) + threadIdx.x;
 
 // run one ray to completion (deterministic kernels, hit-record kernel)
 template <bool STATS>
 __device__ __forceinline__ void trace(Trav& t, const LtSceneDev& sc, int ignore, float tInit, float epsThr,
-                                      bool anyHit, int* __restrict__ stk, int* __restrict__ list, LtCounters& cnt) {
+                                      bool anyHit, const TravSmem& s, LtCounters& cnt) {
   if (!STATS && sc.tnodes != nullptr) {  // small scene: stackless traversal of the threaded tree, same tests
     trav_begin_threaded(t, sc, ignore, tInit, anyHit);
-    const unsigned fifoAddr = (unsigned)__cvta_generic_to_shared(list);
-    while (!trav_iter_threaded(t, sc, fifoAddr, epsThr, LT_MAX_BATCH, LT_MAX_BATCH)) {
+    while (!trav_iter_threaded(t, sc, s.fifoAddr, epsThr, LT_MAX_BATCH, LT_MAX_BATCH)) {
     }
     return;
   }
   trav_begin<STATS>(t, sc, ignore, tInit, anyHit, cnt);
   while (t.cur != LT_DONE) {
-    int n = trav_collect<STATS>(t, sc, stk, list, LT_MAX_BATCH, cnt);
-    trav_test<STATS>(t, sc, list, n, epsThr, cnt);
+    int n = trav_collect<STATS>(t, sc, s.stk, s.list, LT_MAX_BATCH, cnt);
+    trav_test<STATS>(t, sc, s.list, n, epsThr, cnt);
   }
 }
 
@@ -780,20 +775,20 @@ __device__ __forceinline__ int lens_refract_out(const LtSceneDev& sc, Ray& r, co
 // traceRayThroughLens + refract, basic.cu:79-86,245-298 (operation order: oracle/notes_fma_order.md)
 // On entry t holds the primary ray and its hit; on exit the refracted ray and its hit.
 template <bool STATS>
-__device__ void lens_path(const LtSceneDev& sc, Trav& t, float tInit, float epsThr, int* stk, int* list,
-                          float* tstk, bool cull, LtCounters& cnt) {
+__device__ void lens_path(const LtSceneDev& sc, Trav& t, float tInit, float epsThr, const TravSmem& s, bool cull,
+                          LtCounters& cnt) {
   float r2w;
   {
     const Hit h = t.h;
     const int firstPrim = lens_refract_in(sc, t.r, h, r2w);
-    if (cull) trace_cull<STATS>(t, sc, firstPrim, tInit, epsThr, stk, tstk, cnt);
-    else trace<STATS>(t, sc, firstPrim, tInit, epsThr, false, stk, list, cnt);
+    if (cull) trace_cull<STATS>(t, sc, firstPrim, tInit, epsThr, s, cnt);
+    else trace<STATS>(t, sc, firstPrim, tInit, epsThr, false, s, cnt);
   }
   {
     const Hit h = t.h;
     const int secondPrim = lens_refract_out(sc, t.r, h, r2w);
-    if (cull) trace_cull<STATS>(t, sc, secondPrim, tInit, epsThr, stk, tstk, cnt);
-    else trace<STATS>(t, sc, secondPrim, tInit, epsThr, false, stk, list, cnt);
+    if (cull) trace_cull<STATS>(t, sc, secondPrim, tInit, epsThr, s, cnt);
+    else trace<STATS>(t, sc, secondPrim, tInit, epsThr, false, s, cnt);
   }
 }
 

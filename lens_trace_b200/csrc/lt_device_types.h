@@ -19,6 +19,15 @@ constexpr int LT_DEV_FLAG_STATS_TRACED = 1 << 7;
 #define LT_BLOCK 128     // threads per block of the library's traversal kernels
 #define LT_MAX_BATCH 16  // leaf-list entries per thread (shared memory: [LT_MAX_BATCH][LT_BLOCK] ints)
 
+// stack levels a stack traversal reserves for a tree of `stackDepth` levels (LtSceneDev, or the planner's scene facts)
+template <class Scene>
+__host__ __device__ inline int lt_stack_levels(const Scene& s) { return s.stackDepth < 1 ? 1 : s.stackDepth; }
+// Dynamic shared memory of a traversal, ints laid out [level][thread]: `levels` stack levels, the LT_MAX_BATCH-entry
+// leaf list / FIFO, and for culled launches `levels` entry distances (lt_device.cuh: LT_TRAV_SMEM carves it)
+__host__ __device__ inline unsigned lt_traversal_smem(int levels, unsigned threads, bool cull) {
+  return (unsigned)(levels * (cull ? 2 : 1) + LT_MAX_BATCH) * threads * 4u;
+}
+
 struct LtLaunch {
   int kernel;        // lt_kernel
   int kernelMode;    // 0 linear, 1 tile

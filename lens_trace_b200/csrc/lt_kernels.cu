@@ -22,7 +22,7 @@
 template <bool STATS>
 __global__ void __launch_bounds__(LT_BLOCK) k_flat(LtSceneDev sc, LtLaunch L, float* __restrict__ out,
                                                    LtCounters* gcnt) {
-  LT_SMEM_POINTERS(sc)
+  LT_TRAV_SMEM(s, lt_stack_levels(sc))
   int px, py;
   if (!thread_pixel(L.width, L.height, px, py)) return;
   LtCounters cnt = {0, 0, 0};
@@ -32,8 +32,8 @@ __global__ void __launch_bounds__(LT_BLOCK) k_flat(LtSceneDev sc, LtLaunch L, fl
   const float tInit = lt_tinit(L.kernel), epsThr = lt_eps(L.kernel);
   float color[3] = {0.0f, 0.0f, 0.0f};
   const bool cull = (L.flags & LT_DEV_FLAG_CULL) != 0;
-  if (cull) trace_cull<STATS>(t, sc, -1, tInit, epsThr, stk, tstk, cnt);
-  else trace<STATS>(t, sc, -1, tInit, epsThr, false, stk, list, cnt);
+  if (cull) trace_cull<STATS>(t, sc, -1, tInit, epsThr, s, cnt);
+  else trace<STATS>(t, sc, -1, tInit, epsThr, false, s, cnt);
   if (t.h.hit == 1) {
     if (L.kernel == LT_DEV_KERNEL_CUSTOM_BARY) {  // custom_opencl.cl:240
       color[0] = t.h.u;
@@ -42,7 +42,7 @@ __global__ void __launch_bounds__(LT_BLOCK) k_flat(LtSceneDev sc, LtLaunch L, fl
     } else {  // basic.cu:312-326
       const RefMaterial* mat = sc.mats + sc.prims[t.h.prim].materialIndex;
       if (mat->dissolve < 1.0f) {
-        lens_path<STATS>(sc, t, tInit, epsThr, stk, list, tstk, cull, cnt);
+        lens_path<STATS>(sc, t, tInit, epsThr, s, cull, cnt);
         if (t.h.hit == 1) mat = sc.mats + sc.prims[t.h.prim].materialIndex;
       }
       color[0] = mat->diffuse[0];
@@ -76,11 +76,7 @@ __global__ void __launch_bounds__(LT_BLOCK) k_flat(LtSceneDev sc, LtLaunch L, fl
 // tests compare the two).
 __global__ void __launch_bounds__(LT_BLOCK) k_flat_stream(LtSceneDev sc, LtLaunch L, float* __restrict__ out,
                                                           int* __restrict__ work) {
-  extern __shared__ int smemStack[];
-  int* stk = smemStack + threadIdx.x;
-  int* list = smemStack + lt_stack_levels(sc) * LT_BLOCK + threadIdx.x;
-  const unsigned stkAddr = (unsigned)__cvta_generic_to_shared(stk);
-  const unsigned fifoAddr = (unsigned)__cvta_generic_to_shared(list);
+  LT_TRAV_SMEM(s, lt_stack_levels(sc))
   const unsigned lane = threadIdx.x & 31u;
   const float tInit = lt_tinit(L.kernel), epsThr = lt_eps(L.kernel);
   const float camC = cosf(L.cam.yaw), camS = sinf(L.cam.yaw);
@@ -104,7 +100,7 @@ __global__ void __launch_bounds__(LT_BLOCK) k_flat_stream(LtSceneDev sc, LtLaunc
     int ignore = -1;
     for (int stage = 0; stage < 3; stage++) {  // 0 camera ray, 1 and 2 the rays through a lens (basic.cu:245-298)
       trav_begin<false>(t, sc, ignore, tInit, false, cnt);
-      while (!trav_iter_lean<false>(t, sc, stkAddr, fifoAddr, epsThr, kLeanNodeSteps, kLeanTriTests, cnt)) {
+      while (!trav_iter_lean<false>(t, sc, s.stkAddr, s.fifoAddr, epsThr, kLeanNodeSteps, kLeanTriTests, cnt)) {
       }
       const Hit h = t.h;
       if (stage == 0) {
@@ -152,9 +148,8 @@ constexpr int kPathRefillLanes = 4;
 template <bool STATS>
 __global__ void __launch_bounds__(LT_BLOCK) k_path(LtSceneDev sc, LtLaunch L, float* __restrict__ out,
                                                    LtCounters* gcnt) {
-  LT_SMEM_POINTERS(sc)
-  (void)tstk;  // the persistent megakernel does not cull (LT_FLAG_CULL selects the wavefront pipeline)
-  const unsigned fifoAddr = (unsigned)__cvta_generic_to_shared(list);
+  // the persistent megakernel does not cull (LT_FLAG_CULL selects the wavefront pipeline)
+  LT_TRAV_SMEM(s, lt_stack_levels(sc))
   int px, py;
   bool alive = thread_pixel(L.width, L.height, px, py);
   LtCounters cnt = {0, 0, 0};
@@ -237,10 +232,10 @@ __global__ void __launch_bounds__(LT_BLOCK) k_path(LtSceneDev sc, LtLaunch L, fl
       if (waiting && __popc(active) < kPathRefillLanes) break;
       if (traversing) {
         if (threaded) {
-          traversing = !trav_iter_threaded(t, sc, fifoAddr, pc.epsThr, kThreadedNodeSteps, kThreadedTriTests);
+          traversing = !trav_iter_threaded(t, sc, s.fifoAddr, pc.epsThr, kThreadedNodeSteps, kThreadedTriTests);
         } else {
-          int n = trav_collect<STATS>(t, sc, stk, list, LT_MAX_BATCH, cnt);
-          trav_test<STATS>(t, sc, list, n, pc.epsThr, cnt);
+          int n = trav_collect<STATS>(t, sc, s.stk, s.list, LT_MAX_BATCH, cnt);
+          trav_test<STATS>(t, sc, s.list, n, pc.epsThr, cnt);
           traversing = (t.cur != LT_DONE);
         }
       }
@@ -255,15 +250,15 @@ __global__ void __launch_bounds__(LT_BLOCK) k_path(LtSceneDev sc, LtLaunch L, fl
 __global__ void __launch_bounds__(LT_BLOCK) k_primary_hits(LtSceneDev sc, RefCamera cam, int kernel, int flags,
                                                            int width, int height, int* __restrict__ ids,
                                                            int* __restrict__ hit, float* __restrict__ tuv) {
-  LT_SMEM_POINTERS(sc)
+  LT_TRAV_SMEM(s, lt_stack_levels(sc))
   int px, py;
   if (!thread_pixel(width, height, px, py)) return;
   LtCounters cnt = {0, 0, 0};
   float fx, fy;
   Trav t;
   t.r = camera_ray(cam, px, py, width, height, fx, fy);
-  if (flags & LT_DEV_FLAG_CULL) trace_cull<false>(t, sc, -1, lt_tinit(kernel), lt_eps(kernel), stk, tstk, cnt);
-  else trace<false>(t, sc, -1, lt_tinit(kernel), lt_eps(kernel), false, stk, list, cnt);
+  if (flags & LT_DEV_FLAG_CULL) trace_cull<false>(t, sc, -1, lt_tinit(kernel), lt_eps(kernel), s, cnt);
+  else trace<false>(t, sc, -1, lt_tinit(kernel), lt_eps(kernel), false, s, cnt);
   const Hit h = t.h;
   long long i = (long long)py * width + px;
   if (ids) ids[i] = h.prim;
@@ -442,7 +437,7 @@ int lt_launch_reflatten(const RefNode* dNodes, int nodeCount, const RefPrim* dPr
 }
 
 // The culled mode on a tree deeper than 40 levels asks for up to (2 * 64 + 16) * 512 = 73 728 bytes.
-#define LT_MAX_TRAVERSAL_SMEM ((2 * 64 + LT_MAX_BATCH) * LT_BLOCK * (int)sizeof(int))
+static const int kMaxTraversalSmem = (int)lt_traversal_smem(64, LT_BLOCK, true);
 void lt_opt_in_traversal_smem(size_t smem) {
   if (smem <= 48 * 1024) return;
   static bool done[64] = {};
@@ -452,9 +447,9 @@ void lt_opt_in_traversal_smem(size_t smem) {
   done[dev] = true;
   const void* const mine[] = {(const void*)k_flat<false>, (const void*)k_flat<true>, (const void*)k_path<false>,
                               (const void*)k_path<true>, (const void*)k_primary_hits, (const void*)k_flat_stream};
-  for (const void* k : mine) cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, LT_MAX_TRAVERSAL_SMEM);
+  for (const void* k : mine) cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxTraversalSmem);
   for (const void* k : lt_wf_traversal_kernels)
-    cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, LT_MAX_TRAVERSAL_SMEM);
+    cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxTraversalSmem);
 }
 
 int lt_launch_render(const LtSceneDev& sc, const LtPlan& plan, const LtLaunch& L, float* dOut, LtCounters* dCounters,

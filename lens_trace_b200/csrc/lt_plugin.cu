@@ -491,8 +491,7 @@ int lt_plugin_launch(LtPlugin* p, int kernelMode, const LtSceneDev* sceneDev, co
   // a plug-in that uses the device API traverses with per-thread stacks / leaf FIFOs in dynamic shared memory
   unsigned smem = 0;
   if (p->sceneSymbol && sceneDev) {
-    const int levels = sceneDev->tnodes ? 0 : (sceneDev->stackDepth < 1 ? 1 : sceneDev->stackDepth);
-    smem = (unsigned)(levels + 16) * (unsigned)(bx * by) * 4u;
+    smem = lt_traversal_smem(sceneDev->tnodes ? 0 : lt_stack_levels(*sceneDev), (unsigned)(bx * by), false);
     if (smem > 200u * 1024u) {
       *err = "plug-in block too large for the traversal stacks of this scene (use a smaller block)";
       return -1;

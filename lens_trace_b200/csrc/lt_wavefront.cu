@@ -65,6 +65,20 @@ __device__ __forceinline__ int wf_pack_path(int path, int stage, int depth) {
   return path | (stage << WF_PATH_BITS) | (depth << (WF_PATH_BITS + 2));
 }
 
+// ray word of a queue entry (rayD.w): the primitive the ray ignores + 1 (0: none) | anyHit << 31
+__device__ __forceinline__ int wf_ray_word(int ignore, bool anyHit) {
+  return (int)((unsigned)(ignore + 1) | (anyHit ? 0x80000000u : 0u));
+}
+__device__ __forceinline__ int wf_ray_ignore(int word) { return (int)((unsigned)word & 0x7fffffffu) - 1; }
+__device__ __forceinline__ bool wf_ray_any_hit(int word) { return ((unsigned)word >> 31) != 0u; }
+
+// hit word of a traced ray (the last word of a hit record, all of a shadow ray's hit): prim | hit << 31
+__device__ __forceinline__ int wf_hit_word(const Hit& h) { return (int)((unsigned)h.prim | (h.hit ? 0x80000000u : 0u)); }
+__device__ __forceinline__ void wf_hit_unpack(int word, Hit& h) {
+  h.prim = (int)((unsigned)word & 0x7fffffffu);
+  h.hit = (int)((unsigned)word >> 31);
+}
+
 __device__ __forceinline__ void pixel_of_path(long long path, int pixels, int width, int& px, int& py, int& frameLocal) {
   frameLocal = (int)(path / pixels);
   int pixel = (int)(path - (long long)frameLocal * pixels);
@@ -109,8 +123,7 @@ template <int OUT>
 __device__ __forceinline__ void queue_store(const LtWfBuffers& B, int dst, int slot, const Ray& r, float tStart,
                                             int ignore, bool anyHit, int path, const WfPayload& pl) {
   B.rayO[dst][slot] = make_float4(r.ox, r.oy, r.oz, tStart);
-  B.rayD[dst][slot] = make_float4(r.dx, r.dy, r.dz,
-                                  __int_as_float((int)((unsigned)(ignore + 1) | (anyHit ? 0x80000000u : 0u))));
+  B.rayD[dst][slot] = make_float4(r.dx, r.dy, r.dz, __int_as_float(wf_ray_word(ignore, anyHit)));
   B.rayPath[dst][slot] = path;
   if (OUT == WF_EXTENSION) wf_dlight(B, dst)[slot] = pl.a.w;
   else B.payA[dst][slot] = pl.a;
@@ -220,8 +233,7 @@ __device__ __forceinline__ void film_of_path(const LtWfPrimary& P, long long pat
 
 __global__ void __launch_bounds__(WF_BLOCK) k_wf_primary_trace(LtSceneDev sc, LtLaunch L, LtWfPrimary P, int pixels,
                                                                int classify) {
-  LT_SMEM_POINTERS(sc)
-  (void)tstk;
+  LT_TRAV_SMEM(s, lt_stack_levels(sc))
   const int pixel = blockIdx.x * blockDim.x + threadIdx.x;
   const bool valid = pixel < pixels;
   bool alive = false;
@@ -231,9 +243,8 @@ __global__ void __launch_bounds__(WF_BLOCK) k_wf_primary_trace(LtSceneDev sc, Lt
     Trav t;
     t.r = camera_ray(L.cam, px, lt_image_row(L, py), L.width, L.fullHeight, fx, fy);
     LtCounters cnt = {0, 0, 0};
-    trace<false>(t, sc, -1, lt_tinit(L.kernel), lt_eps(L.kernel), false, stk, list, cnt);
-    P.hits[pixel] = make_float4(t.h.t, t.h.u, t.h.v,
-                                __int_as_float((int)((unsigned)t.h.prim | (t.h.hit ? 0x80000000u : 0u))));
+    trace<false>(t, sc, -1, lt_tinit(L.kernel), lt_eps(L.kernel), false, s, cnt);
+    P.hits[pixel] = make_float4(t.h.t, t.h.u, t.h.v, __int_as_float(wf_hit_word(t.h)));
     P.film[pixel] = make_float2(fx, fy);
     if (classify) {
       const PathConsts pc = path_consts(L);
@@ -262,7 +273,7 @@ template <bool STATS>
 __global__ void __launch_bounds__(WF_BLOCK) k_wf_primary(LtSceneDev sc, LtLaunch L, LtWfBuffers B, int nf,
                                                          int pixels, int sample, LtCounters* gcnt, LtWfPrimary P,
                                                          int out) {
-  LT_SMEM_POINTERS(sc)
+  LT_TRAV_SMEM(s, lt_stack_levels(sc))
   const float4* __restrict__ primaryHits = P.hits;
   const bool cull = (L.flags & LT_DEV_FLAG_CULL) != 0;  // closest-hit rays skip subtrees behind the current hit
   const PathConsts pc = path_consts(L);
@@ -291,18 +302,16 @@ __global__ void __launch_bounds__(WF_BLOCK) k_wf_primary(LtSceneDev sc, LtLaunch
       if (!STATS && primaryHits != nullptr) {
         film_of_path(P, p, pixels, L, fl, fx, fy);  // the film position camera_ray computes
         float4 hv = primaryHits[(int)(p - (long long)fl * pixels)];
-        unsigned hb = (unsigned)__float_as_int(hv.w);
         t.h.t = hv.x; t.h.u = hv.y; t.h.v = hv.z;
-        t.h.prim = (int)(hb & 0x7fffffffu);
-        t.h.hit = (int)(hb >> 31);
+        wf_hit_unpack(__float_as_int(hv.w), t.h);
         t.r.ox = t.r.oy = t.r.oz = 0.0f;  // a primary hit is shaded from its hit record alone (shade_step, ST_PRIMARY)
         t.r.dx = t.r.dy = 0.0f;
         t.r.dz = 1.0f;
       } else {
         pixel_of_path(p, pixels, L.width, px, py, fl);
         t.r = camera_ray(L.cam, px, lt_image_row(L, py), L.width, L.fullHeight, fx, fy);
-        if (cull) trace_cull<STATS>(t, sc, -1, pc.tInit, pc.epsThr, stk, tstk, cnt);
-        else trace<STATS>(t, sc, -1, pc.tInit, pc.epsThr, false, stk, list, cnt);
+        if (cull) trace_cull<STATS>(t, sc, -1, pc.tInit, pc.epsThr, s, cnt);
+        else trace<STATS>(t, sc, -1, pc.tInit, pc.epsThr, false, s, cnt);
       }
       PathState ps;
       ps.nrm[0] = ps.nrm[1] = ps.nrm[2] = 0.0f;
@@ -351,17 +360,12 @@ template <bool STATS, bool THREADED>
 __global__ void __launch_bounds__(WF_BLOCK) __maxnreg__(STATS ? 64 : 56)
     k_wf_trace(LtSceneDev sc, LtLaunch L, LtWfBuffers B, int q, LtCounters* gcnt, const float4* __restrict__ rayO,
                const float4* __restrict__ rayD, int* __restrict__ hitWords) {
-  extern __shared__ int smemStack[];
-  int* stk = smemStack + threadIdx.x;
-  int* list = smemStack + (THREADED ? 0 : lt_stack_levels(sc) * LT_BLOCK) + threadIdx.x;
-  float* tstk = reinterpret_cast<float*>(smemStack + (lt_stack_levels(sc) + LT_MAX_BATCH) * LT_BLOCK) + threadIdx.x;
+  LT_TRAV_SMEM(s, THREADED ? 0 : lt_stack_levels(sc))
   const bool cull = !THREADED && (L.flags & LT_DEV_FLAG_CULL) != 0;  // closest-hit rays skip subtrees behind the current hit
   const int nFront = B.counts[2 * q];
   const int n = nFront + B.counts[2 * q + 1];  // virtual entries: front region, then the back region
   const float epsThr = lt_eps(L.kernel);
   const unsigned lane = threadIdx.x & 31u;
-  const unsigned stkAddr = (unsigned)__cvta_generic_to_shared(stk);
-  const unsigned fifoAddr = (unsigned)__cvta_generic_to_shared(list);
   LtCounters cnt = {0, 0, 0};
   // rayO / rayD = B.rayO[q] / B.rayD[q], resolved by the host: indexing the by-value struct with a run-time q would
   // go through a local-memory copy and generic loads
@@ -392,9 +396,9 @@ __global__ void __launch_bounds__(WF_BLOCK) __maxnreg__(STATS ? 64 : 56)
           float4 o = rayO[idx], d = rayD[idx];
           t.r.ox = o.x; t.r.oy = o.y; t.r.oz = o.z;
           t.r.dx = d.x; t.r.dy = d.y; t.r.dz = d.z;
-          unsigned bits = (unsigned)__float_as_int(d.w);
-          if (THREADED) trav_begin_threaded(t, sc, (int)(bits & 0x7fffffffu) - 1, o.w, (bits >> 31) != 0u);
-          else trav_begin<STATS>(t, sc, (int)(bits & 0x7fffffffu) - 1, o.w, (bits >> 31) != 0u, cnt);
+          const int rayWord = __float_as_int(d.w);
+          if (THREADED) trav_begin_threaded(t, sc, wf_ray_ignore(rayWord), o.w, wf_ray_any_hit(rayWord));
+          else trav_begin<STATS>(t, sc, wf_ray_ignore(rayWord), o.w, wf_ray_any_hit(rayWord), cnt);
           entry = idx;
           if (t.cur == LT_DONE) {  // missed the root box: finished already
             if (hitWords) hitWords[idx] = 0;
@@ -412,16 +416,16 @@ __global__ void __launch_bounds__(WF_BLOCK) __maxnreg__(STATS ? 64 : 56)
     if (has) {
       bool finished;
       if (THREADED) {
-        finished = trav_iter_threaded(t, sc, fifoAddr, epsThr, kThreadedNodeSteps, kThreadedTriTests);
+        finished = trav_iter_threaded(t, sc, s.fifoAddr, epsThr, kThreadedNodeSteps, kThreadedTriTests);
       } else if (cull && !t.anyHit) {  // a round holds one kind of ray, so this does not split warps
         for (int k = 0; k < 2 * kLeanNodeSteps && t.cur != LT_DONE; k++)
-          trav_step_cull<STATS>(t, sc, stk, tstk, epsThr, cnt);
+          trav_step_cull<STATS>(t, sc, s.stk, s.tstk, epsThr, cnt);
         finished = t.cur == LT_DONE;
       } else {
-        finished = trav_iter_lean<STATS>(t, sc, stkAddr, fifoAddr, epsThr, kLeanNodeSteps, kLeanTriTests, cnt);
+        finished = trav_iter_lean<STATS>(t, sc, s.stkAddr, s.fifoAddr, epsThr, kLeanNodeSteps, kLeanTriTests, cnt);
       }
       if (finished) {
-        const int word = (int)((unsigned)t.h.prim | (t.h.hit ? 0x80000000u : 0u));
+        const int word = wf_hit_word(t.h);
         if (hitWords) hitWords[entry] = word;
         else B.hits[entry] = make_float4(t.h.t, t.h.u, t.h.v, __int_as_float(word));
         entry = -1;
@@ -485,16 +489,14 @@ __global__ void __launch_bounds__(WF_BLOCK, 8) k_wf_shade(LtSceneDev sc, LtLaunc
       r.dx = d.x; r.dy = d.y; r.dz = d.z;
       Hit h;
       h.t = hv.x; h.u = hv.y; h.v = hv.z;
-      unsigned hb = (unsigned)__float_as_int(hv.w);
-      h.prim = (int)(hb & 0x7fffffffu);
-      h.hit = (int)(hb >> 31);
+      wf_hit_unpack(__float_as_int(hv.w), h);
       PathState ps;
       ps.stage = generic ? (word >> WF_PATH_BITS) & 3
                          : (K == WF_FIRST_SHADOW ? ST_SHADOW_DIRECT : (K == WF_SHADOW ? ST_SHADOW_EXT : ST_EXTENSION));
       ps.depth = (int)((unsigned)word >> (WF_PATH_BITS + 2));
       // every ray after the primary one ignores the primitive its path stands on (basic_lighting.cl:271,
       // global_illumination.cl:294,311,350); an extension result sets it or does not read it
-      ps.hitPrim = (int)((unsigned)__float_as_int(d.w) & 0x7fffffffu) - 1;
+      ps.hitPrim = wf_ray_ignore(__float_as_int(d.w));
       const bool shadowStage = ps.stage == ST_SHADOW_DIRECT || ps.stage == ST_SHADOW_EXT;
       const bool lightHit = ps.stage == ST_EXTENSION && is_light(sc, h.prim);
       const bool surfaceHit = ps.stage == ST_EXTENSION && !lightHit && h.hit == 1;
