@@ -291,7 +291,11 @@ int lt_render_plugin(lt_ctx* ctx, lt_scene* scene, const void* camera28, int plu
  *    uint H, uint depth)
  * under the user's own struct names, or the file does not compile.  `#pragma OPENCL FP_CONTRACT OFF` anywhere in the
  * file compiles all of it without contraction (default: a * b + c may fuse, as OpenCL C allows).  A compile error
- * returns LT_ERR_UNSUPPORTED with the NVRTC log, which names the user's file and line.
+ * returns LT_ERR_UNSUPPORTED with the NVRTC log, which names the user's file and line.  A file that says exactly
+ * `#include "lens_trace_b200_device_cl.h"` gets the plug-in device API of lens_trace_b200_device.cuh in OpenCL C
+ * types (lt_trace, lt_occluded, lt_camera_ray, lt_random, lt_sample_light, lt_sample_hemisphere, lt_interpolate, ...)
+ * and is launched with the dynamic shared memory lt_trace needs for its work-group; a work-group whose traversal
+ * stacks do not fit a block returns LT_ERR_INVALID before anything is launched.
  * lt_render_plugin_cl launches it like the reference's OpenCL backend (src/opencl/renderer_opencl.cpp:84-146): one
  * launch per work block, (width / work_block_x) * (height / work_block_y) of them (integer division), global size =
  * the work block, local size = group, currentBlock = the block's index.  A work block of 0 is the whole image in that

@@ -1286,6 +1286,11 @@ int lt_internal_render_plugin(lt_ctx* ctx, lt_scene* scene, const RefCamera& cam
   CK(cudaSetDevice(ctx->device));
   LtPlugin* plugin = ctx->plugins[run.id];
   const bool cl = lt_plugin_is_opencl_c(plugin);
+  std::string err;
+  unsigned smem = 0;
+  // a work-group whose traversal stacks do not fit is refused before anything is launched
+  if (cl && !lt_plugin_smem(plugin, run.kernelMode, &scene->dev, (unsigned)(run.bx * run.by), &smem, &err))
+    return fail(ctx, LT_ERR_INVALID, std::string(who) + ": " + err);
   const size_t floats = (size_t)P.width * P.height * P.depth;
   int rc = ensure_out(ctx, floats);
   if (rc != LT_OK) return rc;
@@ -1312,8 +1317,7 @@ int lt_internal_render_plugin(lt_ctx* ctx, lt_scene* scene, const RefCamera& cam
   std::vector<RefCamera> cams((size_t)P.frames, cam);
   for (int k = 0; k < P.frames; k++) cams[k].frameCount = cam.frameCount + (uint32_t)k * stride;
   CK(cudaMemcpyAsync(ctx->dCamera, cams.data(), sizeof(RefCamera) * cams.size(), cudaMemcpyHostToDevice, ctx->stream));
-  std::string err;
-  if (!cl && lt_plugin_publish_scene(plugin, &scene->dev, ctx->stream, &err) != 0)
+  if (lt_plugin_publish_scene(plugin, &scene->dev, ctx->stream, &err) != 0)
     return fail(ctx, LT_ERR_CUDA, std::string(who) + ": " + err);
   // pixels outside every work block (the remainder of W / wbx and H / wby) read 0; the reference leaves them undefined
   if (cl) CK(cudaMemsetAsync(dFrame, 0, floats * sizeof(float), ctx->stream));
@@ -1327,9 +1331,9 @@ int lt_internal_render_plugin(lt_ctx* ctx, lt_scene* scene, const RefCamera& cam
   int launches = 0;
   for (int k = 0; k < P.frames; k++) {
     const RefCamera* dCam = ctx->dCamera + k;
-    const int n = cl ? lt_plugin_launch_cl(plugin, run.kernelMode, scene->dNodes, scene->dPrims, scene->dMats,
-                                           scene->dLights, dCam, dFrame, P.width, P.height, P.depth, run.wbx, run.wby,
-                                           run.bx, run.by, ctx->stream, &err)
+    const int n = cl ? lt_plugin_launch_cl(plugin, run.kernelMode, &scene->dev, scene->dNodes, scene->dPrims,
+                                           scene->dMats, scene->dLights, dCam, dFrame, P.width, P.height, P.depth,
+                                           run.wbx, run.wby, run.bx, run.by, ctx->stream, &err)
                      : (lt_plugin_launch(plugin, run.kernelMode, &scene->dev, scene->dNodes, scene->dPrims, scene->dMats,
                                          scene->dLights, dCam, dFrame, P.width, P.height, P.depth, run.bx, run.by,
                                          ctx->stream, &err) == 0 ? 1 : -1);
@@ -1450,9 +1454,9 @@ extern "C" int lt_render_plugin_frames(lt_ctx* ctx, lt_scene* scene, const void*
 
 extern "C" int64_t lt_debug_translate_cl(const char* text, char* out, uint64_t out_bytes, int32_t* contract_off) {
   if (!text) return fail(nullptr, LT_ERR_INVALID, "lt_debug_translate_cl: NULL text");
-  bool off = false;
+  bool off = false, deviceApi = false;
   std::vector<std::pair<std::string, int>> kernels;
-  std::string t = lt_cl_translate(text, &off, &kernels);
+  std::string t = lt_cl_translate(text, &off, &deviceApi, &kernels);
   if (contract_off) *contract_off = off ? 1 : 0;
   if (out && out_bytes > t.size()) memcpy(out, t.c_str(), t.size() + 1);
   return (int64_t)t.size() + 1;

@@ -103,11 +103,16 @@ int lt_plugin_launch(LtPlugin* p, int kernelMode, const LtSceneDev* sceneDev, co
 // OpenCL backend launches them
 bool lt_plugin_is_opencl_c(const LtPlugin* p);
 bool lt_plugin_compile_cl_only(const char* path, std::string* err);  // NVRTC only, no driver
-std::string lt_cl_translate(const std::string& src, bool* contractOff, std::vector<std::pair<std::string, int>>* kernels);
+std::string lt_cl_translate(const std::string& src, bool* contractOff, bool* deviceApi,
+                            std::vector<std::pair<std::string, int>>* kernels);
 bool lt_plugin_cl_shape(int width, int height, int* wbx, int* wby, int* gx, int* gy, std::string* err);
-int lt_plugin_launch_cl(LtPlugin* p, int kernelMode, const void* dNodes, const void* dPrims, const void* dMats,
-                        const void* dLights, const void* dCamera, float* dOut, int width, int height, int depth, int wbx,
-                        int wby, int gx, int gy, cudaStream_t stream, std::string* err);
+// dynamic shared memory of a block of `threads` threads of a plug-in on a scene (the device API's traversal stacks);
+// false with `err` set when they do not fit
+bool lt_plugin_smem(const LtPlugin* p, int kernelMode, const LtSceneDev* sceneDev, unsigned threads, unsigned* smem,
+                    std::string* err);
+int lt_plugin_launch_cl(LtPlugin* p, int kernelMode, const LtSceneDev* sceneDev, const void* dNodes, const void* dPrims,
+                        const void* dMats, const void* dLights, const void* dCamera, float* dOut, int width, int height,
+                        int depth, int wbx, int wby, int gx, int gy, cudaStream_t stream, std::string* err);
 // k_plugin_accumulate (lt_kernels.cu): folds one plug-in frame (`sample`) into the accumulator `acc` with FrameSink, as
 // L.accumMode / L.accumWeight / L.cam.frameCount say; 3 channels per pixel at stride L.depth
 int lt_launch_plugin_accumulate(const LtLaunch& L, const float* sample, float* acc, int smCount, cudaStream_t stream);

@@ -5,6 +5,9 @@
 // device constant data, the other address-space qualifiers dropped, __kernel -> __device__, __local -> an undefined
 // name, `#pragma OPENCL` lines dropped), and places the user's text inside namespace lt_opencl,
 // after this header.  Entities without an execution-space qualifier are device code (-default-device).
+// A file that includes lens_trace_b200_device_cl.h (the plug-in device API in OpenCL C types) has
+// lens_trace_b200_device.cuh compiled at global scope before this header, and the OpenCL C view of it inside
+// namespace lt_opencl after this header, ahead of the user's text.
 //
 // What is provided (OpenCL C 1.2, the part the reference's kernel files use):
 //   - address spaces __global __constant __private (and the spellings without underscores), __kernel / kernel

@@ -104,8 +104,8 @@ struct LtPlugin {
   CUdeviceptr sceneSymbol = 0;  // address of the plug-in's `lt_scene` constant, 0 if it does not use the device API
 };
 
-// texts of include/lens_trace_b200_device.cuh, lt_device.cuh, lt_device_types.h and lt_opencl_c.cuh, handed to NVRTC
-// as headers
+// texts of include/lens_trace_b200_device.cuh, lt_device.cuh, lt_device_types.h, lt_opencl_c.cuh and
+// include/lens_trace_b200_device_cl.h, handed to NVRTC as headers
 #include "lt_device_api_embed.inc"
 
 namespace {
@@ -170,12 +170,16 @@ std::string vector_literals_only(const std::string& line) {
 //     is a compile error at the user's line.  (Macros cannot do this: CUDA's own __global__ expands to `global`.)
 //   - `#pragma OPENCL ...` lines are dropped; `#pragma OPENCL FP_CONTRACT OFF` anywhere turns contraction off for the
 //     whole file (*contractOff)
+//   - `#include "lens_trace_b200_device_cl.h"` is dropped and reported (*deviceApi): cl_source places the device API
+//     ahead of the text; `#include "lens_trace_b200_device.cuh"` becomes an #error that names the OpenCL C header
 //   - the `__kernel void <name>` declarations are recorded with their lines (*kernels)
 // Comments, string and character literals are copied unchanged.
-std::string lt_cl_translate(const std::string& src, bool* contractOff, std::vector<std::pair<std::string, int>>* kernels) {
+std::string lt_cl_translate(const std::string& src, bool* contractOff, bool* deviceApi,
+                            std::vector<std::pair<std::string, int>>* kernels) {
   std::string out;
   out.reserve(src.size() + src.size() / 8);
   *contractOff = false;
+  *deviceApi = false;
   int line = 1, braces = 0, parens = 0;
   bool lineStart = true;
   std::string type;
@@ -208,8 +212,14 @@ std::string lt_cl_translate(const std::string& src, bool* contractOff, std::vect
           words += d[k];
         }
       }
-      if (words.compare(0, 14, "pragma OPENCL ") == 0) {
+      const bool clApi = words == "include \"lens_trace_b200_device_cl.h\"";
+      if (words.compare(0, 14, "pragma OPENCL ") == 0 || clApi) {
         if (words.compare(0, 30, "pragma OPENCL FP_CONTRACT OFF") == 0) *contractOff = true;
+        *deviceApi = *deviceApi || clApi;
+        for (char ch : d)
+          if (ch == '\n') out += '\n';
+      } else if (words == "include \"lens_trace_b200_device.cuh\"") {
+        out += "#error \"an OpenCL C kernel file includes lens_trace_b200_device_cl.h for the device API\"";
         for (char ch : d)
           if (ch == '\n') out += '\n';
       } else {
@@ -310,14 +320,19 @@ std::string quoted(const std::string& s) {
 //   (nodes, primitives, materials, lightContainer, camera, output, uint currentBlock, uint W, uint H, uint depth)
 // as wrappers that convert to the pointer and integer types the user declared; a kernel whose parameters do not take
 // them does not compile.  The call sits on the line of the user's declaration, so the error names it.
+// A file that includes lens_trace_b200_device_cl.h gets the device API first: lens_trace_b200_device.cuh at global
+// scope (so that `lt_scene` keeps the name lt_plugin_module_load looks up), its OpenCL C view inside lt_opencl.
 bool cl_source(const char* path, std::string* program, bool* contractOff, std::vector<std::string>* entries,
                std::string* err) {
   std::string text;
   if (!read_text(path, &text, err)) return false;
   std::vector<std::pair<std::string, int>> kernels;
-  std::string body = lt_cl_translate(text, contractOff, &kernels);
-  std::string p = "#include \"lt_opencl_c.cuh\"\nnamespace lt_opencl {\n#line 1 " + quoted(path) + "\n" + body +
-                  "\n}\n";
+  bool deviceApi = false;
+  std::string body = lt_cl_translate(text, contractOff, &deviceApi, &kernels);
+  std::string p = deviceApi ? "#include \"lens_trace_b200_device.cuh\"\n" : "";
+  p += "#include \"lt_opencl_c.cuh\"\nnamespace lt_opencl {\n";
+  if (deviceApi) p += "#include \"lens_trace_b200_device_cl.h\"\n";
+  p += "#line 1 " + quoted(path) + "\n" + body + "\n}\n";
   bool any = false;
   for (const char* entry : {"linearKernel", "tileKernel"}) {
     int at = 0;
@@ -345,9 +360,10 @@ bool cl_source(const char* path, std::string* program, bool* contractOff, std::v
 bool nvrtc_cubin(const std::string& program, const char* path, bool openclC, bool contractOff, std::vector<char>* cubin,
                  std::string* err) {
   nvrtcProgram prog;
-  const char* headerNames[] = {"lens_trace_b200_device.cuh", "lt_device.cuh", "lt_device_types.h", "lt_opencl_c.cuh"};
-  const char* headerTexts[] = {kEmbedDeviceApi, kEmbedDeviceCode, kEmbedDeviceTypes, kEmbedOpenclC};
-  if (g_api.createProgram(&prog, program.c_str(), path, 4, headerTexts, headerNames) != NVRTC_SUCCESS) {
+  const char* headerNames[] = {"lens_trace_b200_device.cuh", "lt_device.cuh", "lt_device_types.h", "lt_opencl_c.cuh",
+                               "lens_trace_b200_device_cl.h"};
+  const char* headerTexts[] = {kEmbedDeviceApi, kEmbedDeviceCode, kEmbedDeviceTypes, kEmbedOpenclC, kEmbedDeviceApiCl};
+  if (g_api.createProgram(&prog, program.c_str(), path, 5, headerTexts, headerNames) != NVRTC_SUCCESS) {
     *err = "nvrtcCreateProgram failed";
     return false;
   }
@@ -435,12 +451,10 @@ LtPlugin* lt_plugin_module_load(const LtPluginImage& img, std::string* err) {
   }
   g_api.moduleGetFunction(&p->linear, p->module, "linearKernel");
   g_api.moduleGetFunction(&p->tile, p->module, "tileKernel");
-  if (!p->openclC) {
-    size_t bytes = 0;
-    CUdeviceptr addr = 0;
-    if (g_api.moduleGetGlobal(&addr, &bytes, p->module, "lt_scene") == CUDA_SUCCESS && bytes == sizeof(LtSceneDev))
-      p->sceneSymbol = addr;
-  }
+  size_t bytes = 0;
+  CUdeviceptr addr = 0;
+  if (g_api.moduleGetGlobal(&addr, &bytes, p->module, "lt_scene") == CUDA_SUCCESS && bytes == sizeof(LtSceneDev))
+    p->sceneSymbol = addr;
   if (!p->linear && !p->tile) {
     *err = p->path + " exports neither linearKernel nor tileKernel (extern \"C\" __global__)";
     g_api.moduleUnload(p->module);
@@ -469,6 +483,24 @@ int lt_plugin_publish_scene(LtPlugin* p, const LtSceneDev* sceneDev, cudaStream_
   return 0;
 }
 
+// Dynamic shared memory of a launch of plug-in `p`'s kernelMode entry point with `threads` threads per block on the
+// scene `sceneDev`: a plug-in that uses the device API traverses with per-thread stacks / leaf FIFOs there (lt_trace),
+// any other gets none.  Above 48 KB the entry point's limit is raised to the size.  Returns false with `err` set when
+// the stacks do not fit a block.
+bool lt_plugin_smem(const LtPlugin* p, int kernelMode, const LtSceneDev* sceneDev, unsigned threads, unsigned* smem,
+                    std::string* err) {
+  *smem = 0;
+  if (!p->sceneSymbol || !sceneDev) return true;
+  *smem = lt_traversal_smem(sceneDev->tnodes ? 0 : lt_stack_levels(*sceneDev), threads, false);
+  if (*smem > 200u * 1024u) {
+    *err = "plug-in block too large for the traversal stacks of this scene (use a smaller block)";
+    return false;
+  }
+  CUfunction fn = kernelMode ? p->tile : p->linear;
+  if (fn && *smem > 48u * 1024u) g_api.funcSetAttribute(fn, CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES, (int)*smem);
+  return true;
+}
+
 // Launch shape of the reference: grid = ceil(W/bx) x ceil(H/by), block = bx x by (32x1 for MAX_FIT,
 // src/cuda/renderer_cuda.cpp:74-88).  sceneDev (published by lt_plugin_publish_scene) sizes the traversal stacks.
 // Returns 0, or -1 with `err` set.
@@ -488,16 +520,8 @@ int lt_plugin_launch(LtPlugin* p, int kernelMode, const LtSceneDev* sceneDev, co
     *err = "plug-in block size exceeds 1024 threads";
     return -1;
   }
-  // a plug-in that uses the device API traverses with per-thread stacks / leaf FIFOs in dynamic shared memory
   unsigned smem = 0;
-  if (p->sceneSymbol && sceneDev) {
-    smem = lt_traversal_smem(sceneDev->tnodes ? 0 : lt_stack_levels(*sceneDev), (unsigned)(bx * by), false);
-    if (smem > 200u * 1024u) {
-      *err = "plug-in block too large for the traversal stacks of this scene (use a smaller block)";
-      return -1;
-    }
-    if (smem > 48u * 1024u) g_api.funcSetAttribute(fn, CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES, (int)smem);
-  }
+  if (!lt_plugin_smem(p, kernelMode, sceneDev, (unsigned)(bx * by), &smem, err)) return -1;
   void* args[] = {(void*)&dNodes, (void*)&dPrims, (void*)&dMats, (void*)&dLights, (void*)&dCamera,
                   (void*)&dOut,   (void*)&width,  (void*)&height, (void*)&depth};
   CUresult rc = g_api.launchKernel(fn, (unsigned)((width + bx - 1) / bx), (unsigned)((height + by - 1) / by), 1,
@@ -546,23 +570,25 @@ bool lt_plugin_cl_shape(int width, int height, int* wbx, int* wby, int* gx, int*
 
 // The reference's OpenCL launch loop (renderer_opencl.cpp:84-146, restated in oracle/cl_shim/ref_cl_host.cpp): one
 // NDRange per work block, global size = the work block, local size = the group, currentBlock = the block's index, for
-// (W / wbx) * (H / wby) blocks.  Arguments as normalised by lt_plugin_cl_shape.  Returns launches made, or -1 with
-// `err` set.
-int lt_plugin_launch_cl(LtPlugin* p, int kernelMode, const void* dNodes, const void* dPrims, const void* dMats,
-                        const void* dLights, const void* dCamera, float* dOut, int width, int height, int depth, int wbx,
-                        int wby, int gx, int gy, cudaStream_t stream, std::string* err) {
+// (W / wbx) * (H / wby) blocks.  Arguments as normalised by lt_plugin_cl_shape; sceneDev sizes the traversal stacks of
+// a file that uses the device API, as in lt_plugin_launch.  Returns launches made, or -1 with `err` set.
+int lt_plugin_launch_cl(LtPlugin* p, int kernelMode, const LtSceneDev* sceneDev, const void* dNodes, const void* dPrims,
+                        const void* dMats, const void* dLights, const void* dCamera, float* dOut, int width, int height,
+                        int depth, int wbx, int wby, int gx, int gy, cudaStream_t stream, std::string* err) {
   CUfunction fn = kernelMode ? p->tile : p->linear;
   if (!fn) {
     *err = p->path + (kernelMode ? " has no tileKernel" : " has no linearKernel");
     return -1;
   }
+  unsigned smem = 0;
+  if (!lt_plugin_smem(p, kernelMode, sceneDev, (unsigned)(gx * gy), &smem, err)) return -1;
   const unsigned blocks = (unsigned)(width / wbx) * (unsigned)(height / wby);
   unsigned block = 0, w = (unsigned)width, h = (unsigned)height, d = (unsigned)depth;
   void* args[] = {(void*)&dNodes, (void*)&dPrims, (void*)&dMats, (void*)&dLights, (void*)&dCamera,
                   (void*)&dOut,   (void*)&block,  (void*)&w,     (void*)&h,       (void*)&d};
   for (block = 0; block < blocks; block++) {
-    CUresult rc = g_api.launchKernel(fn, (unsigned)(wbx / gx), (unsigned)(wby / gy), 1, (unsigned)gx, (unsigned)gy, 1, 0,
-                                     (CUstream)stream, args, nullptr);
+    CUresult rc = g_api.launchKernel(fn, (unsigned)(wbx / gx), (unsigned)(wby / gy), 1, (unsigned)gx, (unsigned)gy, 1,
+                                     smem, (CUstream)stream, args, nullptr);
     if (rc != CUDA_SUCCESS) {
       *err = "cuLaunchKernel failed for plug-in " + p->path + " (CUresult " + std::to_string((int)rc) + ")";
       return -1;
