@@ -237,11 +237,22 @@ int lt_debug_build_threaded_pruned(const void* nodes, uint64_t node_bytes, void*
  * prim_count.  out_records (16 * node_count * 32 bytes of room): the eight full copies, then the eight pruned copies
  * (*out_stride records each; skip links absolute, from record 8 * node_count).  When every leaf box lies inside all
  * its ancestors' boxes (bounds finite, lo <= hi, no primitive linked twice, inner root), the pruned copies are those
- * of a traversal tree: a SAH tree over the reference's leaves that reaches the same leaves in another order.  Then
+ * of a traversal tree: a tree over the reference's leaves, built for the cost of the pruned walk
+ * (lt_debug_traversal_tree_costs), that reaches the same leaves in another order.  Then
  * *out_traversal = 1 and out_rank (8 * prim_count int32) receives the tie-break table rank[o][p] (LtSceneDev::rank);
  * otherwise *out_traversal = 0, the pruned copies are lt_debug_build_threaded_pruned's and out_rank is not written. */
 int lt_debug_build_traversal_tree(const void* nodes, uint64_t node_bytes, int32_t prim_count, void* out_records,
                                   int32_t* out_stride, int32_t* out_rank, int32_t* out_traversal);
+
+/* Host-only: the traversal tree lt_scene_upload builds for a small tree (see lt_debug_build_traversal_tree), in the
+ * reference's node layout, and the cost model it is chosen by: the expected box tests of the pruned threaded walk per
+ * ray that hits the root box, sum over the kept records r other than the root of SA(nearest kept ancestor of r) /
+ * SA(root).  out_costs[0]: the reference tree's pruned copies; [1], [2], [3]: the candidates over the reference's
+ * leaves -- SAH sweep, PLOC, the better of the two after treelet restructuring --, of which the cheapest is the
+ * traversal tree, written to out_nodes (node_bytes of room).  Without a traversal tree [1..3] are NaN and out_nodes is
+ * not written. */
+int lt_debug_traversal_tree(const void* nodes, uint64_t node_bytes, int32_t prim_count, void* out_nodes,
+                            double* out_costs);
 
 /* Test hook: 1 when the pruned threaded copies of an uploaded scene are a traversal tree, 0 when not (also for
  * scenes without host-built copies), < 0 on error. */

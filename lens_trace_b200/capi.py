@@ -20,7 +20,7 @@ SYMBOLS = [
     "lt_last_stats", "lt_kernel_from_path", "lt_kernel_name", "lt_debug_random", "lt_debug_hemisphere", "lt_debug_build_threaded", "lt_debug_build_threaded_pruned", "lt_debug_scene_full_threaded", "lt_plugin_load", "lt_render_plugin", "lt_render_plugin_cl", "lt_debug_compile_cl", "lt_debug_translate_cl", "lt_primary_hits_flags", "lt_scene_build_lbvh", "lt_scene_build_ploc", "lt_scene_download", "lt_scene_info",
     "lt_debug_gather_peak", "lt_ctx_create_multi", "lt_ctx_device_count", "lt_host_register", "lt_host_unregister", "lt_debug_tile_rows",
     "lt_debug_plan", "lt_debug_ctx_limits", "lt_render_plugin_frames", "lt_debug_build_traversal_tree",
-    "lt_debug_scene_traversal_tree",
+    "lt_debug_scene_traversal_tree", "lt_debug_traversal_tree",
 ]
 
 
@@ -94,6 +94,7 @@ def load():
     lib.lt_debug_build_traversal_tree.argtypes = [C.c_void_p, C.c_uint64, C.c_int32, C.c_void_p, C.POINTER(C.c_int32),
                                                   C.c_void_p, C.POINTER(C.c_int32)]
     lib.lt_debug_scene_traversal_tree.argtypes = [C.c_void_p]
+    lib.lt_debug_traversal_tree.argtypes = [C.c_void_p, C.c_uint64, C.c_int32, C.c_void_p, C.POINTER(C.c_double)]
     lib.lt_debug_ctx_limits.argtypes = [C.c_void_p, C.c_int, C.c_int]
     lib.lt_debug_plan.argtypes = [C.POINTER(RenderParams), C.c_uint64, C.c_int32, C.c_uint64, C.c_int32,
                                   C.POINTER(C.c_int64)]
@@ -425,3 +426,19 @@ def build_traversal_tree(nodes, prim_count):
     pruned["skip"] = np.where(pruned["skip"] == -2147483648, pruned["skip"], pruned["skip"] - 8 * n)
     return {"full": out[:8 * n].reshape(8, n).copy(), "pruned": pruned.reshape(8, k), "stride": k,
             "traversal": trav.value == 1, "rank": rank if trav.value == 1 else None}
+
+
+def traversal_tree(nodes, prim_count):
+    """Host-only: the traversal tree lt_scene_upload builds for a small tree and the costs it is chosen by
+    (lt_debug_traversal_tree), as a dict: "nodes" (the tree in the reference layout, or None when the tree gets none),
+    "reference" (the expected box tests per root-hitting ray of the reference tree's pruned copies), "sah", "ploc" and
+    "restructured" (those of the candidates over the reference's leaves, or None)."""
+    lib = load()
+    nodes = np.ascontiguousarray(nodes)
+    out = np.zeros_like(nodes)
+    cost = (C.c_double * 4)()
+    rc = lib.lt_debug_traversal_tree(nodes.ctypes.data, nodes.nbytes, prim_count, out.ctypes.data, cost)
+    if rc != 0:
+        raise LtError("lt_debug_traversal_tree failed (%d): %s" % (rc, lib.lt_last_error(None).decode()))
+    v = [None if np.isnan(x) else float(x) for x in cost]
+    return {"nodes": None if v[1] is None else out, "reference": v[0], "sah": v[1], "ploc": v[2], "restructured": v[3]}
