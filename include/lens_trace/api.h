@@ -126,6 +126,7 @@ struct AccelerationStructureExplicitProperties {
 
 // Optional, chained on RenderProperties*::pNext.  Lets one render() call take several frames and
 // keep the running mean of examples/accumulator/resources/shaders/accumulator.frag on the device.
+class Camera;
 struct RenderExtensionB200 {
   StructureType sType;     // STRUCTURE_TYPE_RENDER_EXTENSION_B200
   void* pNext;
@@ -140,6 +141,11 @@ struct RenderExtensionB200 {
   // --- multi-GPU (appended: older initialisers leave them 0 = one GPU) ---
   uint32_t deviceCount;    // GPUs 0 .. deviceCount-1 of this process render the call together (0, 1: device 0 only)
   uint32_t splitMode;      // 0 auto, 1 samples (one NCCL all-reduce per call), 2 tiles (blocks of 8 rows, no collective)
+  // --- several views (appended: older initialisers leave them 0 = the one camera pCamera) ---
+  uint32_t viewCount;             // >= 2: render the cameras below instead of pCamera (0, 1: pCamera)
+  Camera* const* ppViewCameras;   // viewCount cameras; pOutputBuffer holds viewCount images, view v at v * w * h * d
+                                  // floats, each accumulated from zero within the call (lt_render_views); deviceCount
+                                  // above 1 deals the views to the devices; built-in kernels only
 };
 
 // ================================================================================================

@@ -179,6 +179,29 @@ int lt_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_rende
 int lt_render_device(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params,
                      float* device_out, int sync);
 
+/* Several camera views of one scene with the same params in one call.  cameras28: view_count >= 1 consecutive
+ * 28-byte camera records.  View v equals lt_accum_reset followed by lt_render with camera v, bit for bit, in every
+ * accum_mode: frame k of view v uses frameCount_v + k * frame_stride, and every view accumulates from zero within the
+ * call.  The context accumulator of lt_render / lt_accum_read / lt_accum_reset is neither read nor changed, with one
+ * exception: on a multi-GPU context view_count == 1 is lt_render (see below).  The views are rendered into a device
+ * buffer the context owns (view_count images); like the wavefront workspace it keeps the largest size asked for until
+ * lt_ctx_destroy.
+ * host_out: view_count * width * height * depth floats, view v at v * width * height * depth (may be NULL).
+ * Every kernel id and flag of lt_render is accepted and means the same; with LT_FLAG_STATS, lt_last_stats counts the
+ * sum over the views.  The views of one call share one wavefront launch when they hold enough paths, otherwise each
+ * runs the megakernel (lt_debug_plan_views).  view_count < 1 or NULL cameras28: LT_ERR_INVALID, nothing launched.
+ * On a multi-GPU context with view_count >= 2, device g renders views g, g+G, ... on its own (no collective);
+ * split_mode must be LT_SPLIT_AUTO (LT_ERR_INVALID otherwise).  There view_count == 1 is lt_render, with its split
+ * and its per-device accumulators.  Synchronous. */
+int lt_render_views(lt_ctx* ctx, lt_scene* scene, const void* cameras28, int view_count,
+                    const lt_render_params* params, float* host_out);
+/* Same, into device memory: device_out holds view_count images on ctx's device and is used as their view_count
+ * accumulators when accum_mode != NONE: slice v equals lt_render_device(camera v, params, slice v) from the same
+ * initial contents.  Asynchronous on the context stream unless sync != 0.  Single-GPU contexts only
+ * (LT_ERR_UNSUPPORTED otherwise, as lt_render_device). */
+int lt_render_views_device(lt_ctx* ctx, lt_scene* scene, const void* cameras28, int view_count,
+                           const lt_render_params* params, float* device_out, int sync);
+
 /* The output buffer of the reference API is the caller's malloc'ed memory (pOutputBuffer, structures.h:62,76).
  * lt_render copies into such pageable memory through its own pinned staging buffer; an application that reuses one
  * buffer for many calls can page-lock it once instead, and the frame then arrives by a single DMA.  Unregister
@@ -281,6 +304,11 @@ int lt_debug_ctx_limits(lt_ctx* ctx, int threaded_max_nodes, int stream_min_node
 #define LT_PLAN_FIELDS 15
 int lt_debug_plan(const lt_render_params* params, uint64_t node_count, int32_t stack_depth, uint64_t total_mem,
                   int32_t sm_count, int64_t* out);
+/* Host-only: the plan of an lt_render_views call of view_count views, as lt_debug_plan (view_count == 1: exactly
+ * lt_debug_plan).  The wavefront's frames per batch then count (view, frame) pairs, and its workspace bytes include
+ * the primary records of every view one batch touches. */
+int lt_debug_plan_views(const lt_render_params* params, int view_count, uint64_t node_count, int32_t stack_depth,
+                        uint64_t total_mem, int32_t sm_count, int64_t* out);
 
 /* --- plug-in kernels: a user-written .cu file with the reference's kernel ABI (extern "C" __global__
  * linearKernel / tileKernel(LinearBVHNode*, Primitive*, Material*, LightContainer*, Camera*, float* out,

@@ -20,7 +20,8 @@ SYMBOLS = [
     "lt_last_stats", "lt_kernel_from_path", "lt_kernel_name", "lt_debug_random", "lt_debug_hemisphere", "lt_debug_build_threaded", "lt_debug_build_threaded_pruned", "lt_debug_scene_full_threaded", "lt_plugin_load", "lt_render_plugin", "lt_render_plugin_cl", "lt_debug_compile_cl", "lt_debug_translate_cl", "lt_primary_hits_flags", "lt_scene_build_lbvh", "lt_scene_build_ploc", "lt_scene_download", "lt_scene_info",
     "lt_debug_gather_peak", "lt_ctx_create_multi", "lt_ctx_device_count", "lt_host_register", "lt_host_unregister", "lt_debug_tile_rows",
     "lt_debug_plan", "lt_debug_ctx_limits", "lt_render_plugin_frames", "lt_debug_build_traversal_tree",
-    "lt_debug_scene_traversal_tree", "lt_debug_traversal_tree",
+    "lt_debug_scene_traversal_tree", "lt_debug_traversal_tree", "lt_render_views", "lt_render_views_device",
+    "lt_debug_plan_views",
 ]
 
 
@@ -79,6 +80,9 @@ def load():
     lib.lt_scene_release.restype = None
     lib.lt_render.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(RenderParams), C.c_void_p]
     lib.lt_render_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(RenderParams), C.c_void_p, C.c_int]
+    lib.lt_render_views.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(RenderParams), C.c_void_p]
+    lib.lt_render_views_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(RenderParams),
+                                           C.c_void_p, C.c_int]
     lib.lt_accum_reset.argtypes = [C.c_void_p]
     lib.lt_accum_read.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64]
     lib.lt_primary_hits.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p,
@@ -98,6 +102,8 @@ def load():
     lib.lt_debug_ctx_limits.argtypes = [C.c_void_p, C.c_int, C.c_int]
     lib.lt_debug_plan.argtypes = [C.POINTER(RenderParams), C.c_uint64, C.c_int32, C.c_uint64, C.c_int32,
                                   C.POINTER(C.c_int64)]
+    lib.lt_debug_plan_views.argtypes = [C.POINTER(RenderParams), C.c_int, C.c_uint64, C.c_int32, C.c_uint64, C.c_int32,
+                                        C.POINTER(C.c_int64)]
     lib.lt_plugin_load.argtypes = [C.c_void_p, C.c_char_p, C.POINTER(C.c_int)]
     lib.lt_render_plugin.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                      C.c_int, C.c_int, C.c_void_p]
@@ -246,6 +252,25 @@ class Context:
         self._check(self.lib.lt_render_device(self.h, scene.h, cam.ctypes.data, C.byref(params),
                                               C.c_void_p(device_ptr), 1 if sync else 0), "lt_render_device")
 
+    def render_views(self, scene, cameras, params, want_output=True):
+        """Several views in one call (lt_render_views): cameras is a sequence of V camera records; returns float32
+        [V, H, W, depth] (view v equals accum_reset + render of camera v) or None."""
+        cams = np.ascontiguousarray(cameras, dtype=L.CAMERA).reshape(-1)
+        out = None
+        if want_output:
+            out = np.empty((cams.size, params.height, params.width, params.depth), dtype=np.float32)
+        self._check(self.lib.lt_render_views(self.h, scene.h, cams.ctypes.data if cams.size else None, cams.size,
+                                             C.byref(params), out.ctypes.data if out is not None else None),
+                    "lt_render_views")
+        return out
+
+    def render_views_device(self, scene, cameras, params, device_ptr, sync=False):
+        """lt_render_views_device: V images at device_ptr (V * H * W * depth floats), slice v the accumulator of view v"""
+        cams = np.ascontiguousarray(cameras, dtype=L.CAMERA).reshape(-1)
+        self._check(self.lib.lt_render_views_device(self.h, scene.h, cams.ctypes.data if cams.size else None, cams.size,
+                                                    C.byref(params), C.c_void_p(device_ptr), 1 if sync else 0),
+                    "lt_render_views_device")
+
     def accum_reset(self):
         self._check(self.lib.lt_accum_reset(self.h), "lt_accum_reset")
 
@@ -373,6 +398,19 @@ def plan(params, node_count, stack_depth, total_mem, sm_count):
     rc = lib.lt_debug_plan(C.byref(params), node_count, stack_depth, total_mem, sm_count, out)
     if rc == ERR_INVALID:
         raise LtError("lt_debug_plan failed (%d): %s" % (rc, lib.lt_last_error(None).decode()))
+    d = dict(zip(PLAN_FIELDS, out))
+    d["error"] = rc
+    d["message"] = lib.lt_last_error(None).decode() if rc else ""
+    return d
+
+
+def plan_views(params, view_count, node_count, stack_depth, total_mem, sm_count):
+    """Host-only: the launch plan of an lt_render_views call of view_count views (lt_debug_plan_views), as plan()."""
+    lib = load()
+    out = (C.c_int64 * len(PLAN_FIELDS))()
+    rc = lib.lt_debug_plan_views(C.byref(params), view_count, node_count, stack_depth, total_mem, sm_count, out)
+    if rc == ERR_INVALID:
+        raise LtError("lt_debug_plan_views failed (%d): %s" % (rc, lib.lt_last_error(None).decode()))
     d = dict(zip(PLAN_FIELDS, out))
     d["error"] = rc
     d["message"] = lib.lt_last_error(None).decode() if rc else ""

@@ -164,8 +164,18 @@ static LtPlan lt_plan_primary_hits(int flags, int width, int height, const LtSce
   return p;
 }
 
+// Views of one call (lt_render_views) share no camera rays, so the frames' threshold does not carry over.  Measured
+// (tools/views_timing.py, profiles/views_timing_b200.txt; NVIDIA B200 at its 1000 W power limit): one-frame 1080p GI
+// views, 4 bounces, on the Cornell box, ms per view of the megakernel (one launch per view) against the wavefront over
+// the views: V = 1 (2 073 600 paths) 0.705 against 0.787, V = 2 (4 147 200) 0.716 against 0.551, V = 4 0.799 against
+// 0.485, V = 8 0.822 against 0.447, V = 16 0.796 against 0.403.  The crossover lies between 2.1 M and 4.1 M paths.
+// The lighting kernels keep their factor of 4 (not measured for views).
+static const long long kViewsMinPaths = 3ll << 20;
+
+// views: a call of several views (lt_render_views) runs its (view, frame) pairs through one wavefront launch, or one
+// megakernel launch per view
 static LtPlan lt_plan_render(const LtLaunch& L, const LtSceneFacts& s, size_t totalMem, int smCount,
-                             const LtLimits& lim) {
+                             const LtLimits& lim, int views = 1) {
   LtPlan p = {};
   p.error = LT_OK;
   p.stats = (L.flags & LT_FLAG_STATS) != 0;
@@ -179,10 +189,11 @@ static LtPlan lt_plan_render(const LtLaunch& L, const LtSceneFacts& s, size_t to
     // and for the two-ray lighting kernels on small scenes, its per-round launches and state traffic lose.  Second
     // measurement (shared camera rays, overlapped batches): the two-ray lighting kernels on a small scene win too
     // once a launch holds several batches (64 frames at 1080p: 1.31x); the 25-sample kernels stay on k_path
-    const long long minPaths = 1ll << 23;
+    const long long minPaths = views > 1 ? kViewsMinPaths : 1ll << 23;
     const long long need = (isGI || s.nodeCount > 100000) ? minPaths : 4 * minPaths;
     const bool forced = (L.flags & (LT_FLAG_WAVEFRONT | LT_FLAG_CULL)) != 0;
-    bool wavefront = forced || (pixels * L.frames >= need && L.kernel != LT_KERNEL_GI25 &&
+    const long long pairs = (long long)L.frames * views;  // (view, frame) pairs, view-major
+    bool wavefront = forced || (pixels * pairs >= need && L.kernel != LT_KERNEL_GI25 &&
                                 L.kernel != LT_KERNEL_LIGHTING25);
     // A queue entry carries the bounce depth in 5 bits (wf_pack_path): deeper bounce caps stay on the megakernel,
     // which is the same arithmetic per path (0 = the reference constant 16).  It carries its path id in 25 bits:
@@ -206,12 +217,12 @@ static LtPlan lt_plan_render(const LtLaunch& L, const LtSceneFacts& s, size_t to
       if (cap > memCap) cap = memCap;
       int batchFrames = (int)(cap / pixels);
       if (batchFrames < 1) batchFrames = 1;
-      if (batchFrames > L.frames) batchFrames = L.frames;
+      if (batchFrames > pairs) batchFrames = (int)pairs;
       // Two consecutive batches overlap on two streams (the trace kernel of one beside the shade kernel of the other:
       // L1 data pipe vs DRAM): half-size batches, one workspace each -- same memory.  LT_FLAG_SERIAL: one stream,
       // kernels run one at a time.  Measured: reserving room on the SMs for the other batch's blocks (fewer
       // persistent trace blocks) does not pay, nor do 3 or 4 batches in flight (profiles/r2u_overlap_sweep.txt).
-      p.streams = !(L.flags & (LT_FLAG_SERIAL | LT_FLAG_STATS)) && L.frames >= 2 ? 2 : 1;
+      p.streams = !(L.flags & (LT_FLAG_SERIAL | LT_FLAG_STATS)) && pairs >= 2 ? 2 : 1;
       batchFrames = (batchFrames + p.streams - 1) / p.streams;
       long long perBatch = (1ll << 25) / pixels;  // a queue entry carries its path id in 25 bits
       if (perBatch < 1) perBatch = 1;
@@ -220,8 +231,13 @@ static LtPlan lt_plan_render(const LtLaunch& L, const LtSceneFacts& s, size_t to
       p.rounds = isGI ? 2 + 2 * (L.maxRayDepth > 0 ? L.maxRayDepth : 16) : 2;
       p.sharedPrimary = !p.stats && !p.cull;  // the exact, uncounted pipelines
       p.classify = p.sharedPrimary && p.samplesPerFrame == 1;
-      p.workspaceBytes = lt_wf_workspace_bytes_padded((long long)p.batchFrames * pixels) * (size_t)p.streams +
-                         lt_wf_primary_hits_bytes(pixels);
+      // primary records: one set per launch; with views, one set per view a batch touches, per batch workspace
+      size_t records = lt_wf_primary_hits_bytes(pixels);
+      if (views > 1)
+        records = p.sharedPrimary ? lt_wf_view_records_bytes(pixels, lt_wf_views_per_batch(p.batchFrames, L.frames,
+                                                                                            views)) * (size_t)p.streams
+                                  : 0;
+      p.workspaceBytes = lt_wf_workspace_bytes_padded((long long)p.batchFrames * pixels) * (size_t)p.streams + records;
     }
   }
   // camera rays and one shadow ray per hit: the two lighting kernels on the megakernel
@@ -311,6 +327,8 @@ extern "C" void lt_ctx_destroy(lt_ctx* ctx) {
   if (ctx->wfWorkspace) cudaFree(ctx->wfWorkspace);
   if (ctx->dCamera) cudaFree(ctx->dCamera);
   if (ctx->dSample) cudaFree(ctx->dSample);
+  if (ctx->dViews) cudaFree(ctx->dViews);
+  if (ctx->dViewFrameCounts) cudaFree(ctx->dViewFrameCounts);
   delete ctx->copyPool;
   if (ctx->stage) cudaFreeHost(ctx->stage);
   for (cudaEvent_t e : ctx->stageEvents) cudaEventDestroy(e);
@@ -1484,20 +1502,30 @@ static LtSceneDev scene_for_plan(const lt_scene* s, const LtPlan& plan) {
   return d;
 }
 
-extern "C" int lt_debug_plan(const lt_render_params* params, uint64_t node_count, int32_t stack_depth,
-                             uint64_t total_mem, int32_t sm_count, int64_t* out) {
-  if (!params || !out || node_count < 1 || node_count > 0x7fffffffull || sm_count < 1)
-    return fail(nullptr, LT_ERR_INVALID, "lt_debug_plan: bad arguments");
+static int debug_plan(const char* who, const lt_render_params* params, int views, uint64_t node_count,
+                      int32_t stack_depth, uint64_t total_mem, int32_t sm_count, int64_t* out) {
+  if (!params || !out || views < 1 || node_count < 1 || node_count > 0x7fffffffull || sm_count < 1)
+    return fail(nullptr, LT_ERR_INVALID, std::string(who) + ": bad arguments");
   LtLaunch L = {};
   if (int rc = launch_from_params(nullptr, params, &L)) return rc;
   const LtLimits lim;
   const LtSceneFacts s = {(int)node_count, stack_depth, lt_plan_threaded_copies((int)node_count, total_mem, lim)};
-  const LtPlan p = lt_plan_render(L, s, total_mem, sm_count, lim);
+  const LtPlan p = lt_plan_render(L, s, total_mem, sm_count, lim, views);
   const int64_t v[LT_PLAN_FIELDS] = {p.pipeline, p.tree, p.stats, p.cull, p.batchFrames, p.streams, p.rounds,
                                      p.samplesPerFrame, p.sharedPrimary, p.classify, (int64_t)p.smemStack,
                                      (int64_t)p.smemTrace, p.blocksPerSm, p.grid, (int64_t)p.workspaceBytes};
   memcpy(out, v, sizeof v);
   return p.error != LT_OK ? fail(nullptr, p.error, p.message) : LT_OK;
+}
+
+extern "C" int lt_debug_plan(const lt_render_params* params, uint64_t node_count, int32_t stack_depth,
+                             uint64_t total_mem, int32_t sm_count, int64_t* out) {
+  return debug_plan("lt_debug_plan", params, 1, node_count, stack_depth, total_mem, sm_count, out);
+}
+
+extern "C" int lt_debug_plan_views(const lt_render_params* params, int view_count, uint64_t node_count,
+                                   int32_t stack_depth, uint64_t total_mem, int32_t sm_count, int64_t* out) {
+  return debug_plan("lt_debug_plan_views", params, view_count, node_count, stack_depth, total_mem, sm_count, out);
 }
 
 extern "C" int lt_debug_ctx_limits(lt_ctx* ctx, int threaded_max_nodes, int stream_min_nodes) {
@@ -1522,9 +1550,11 @@ int lt_internal_ensure_out(lt_ctx* ctx, size_t floats) {
   return LT_OK;
 }
 
-static int render_common(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, float* dOut, bool sync) {
+// cams: the cameras of a call of several views (viewCount >= 2, view v into dOut + v * W * H * depth); nullptr: L.cam
+static int render_common(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, float* dOut, bool sync,
+                         const RefCamera* cams = nullptr, int viewCount = 1) {
   CK(cudaSetDevice(ctx->device));
-  LtPlan plan = lt_plan_render(L, scene_facts(scene), ctx->totalMem, ctx->stats.sm_count, ctx->limits);
+  LtPlan plan = lt_plan_render(L, scene_facts(scene), ctx->totalMem, ctx->stats.sm_count, ctx->limits, viewCount);
   if (plan.error != LT_OK) return fail(ctx, plan.error, plan.message);
   const bool stats = plan.stats;
   if (stats) CK(cudaMemsetAsync(ctx->dCounters, 0, sizeof(LtCounters), ctx->stream));
@@ -1538,7 +1568,7 @@ static int render_common(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, float*
       // not a fallback to other arithmetic: the megakernel is the same path per pixel
       LtLaunch mega = L;
       mega.flags |= LT_FLAG_MEGAKERNEL;
-      plan = lt_plan_render(mega, scene_facts(scene), ctx->totalMem, ctx->stats.sm_count, ctx->limits);
+      plan = lt_plan_render(mega, scene_facts(scene), ctx->totalMem, ctx->stats.sm_count, ctx->limits, viewCount);
     } else {
       ctx->wfBytes = plan.workspaceBytes;
     }
@@ -1555,13 +1585,40 @@ static int render_common(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, float*
   // per-kernel times are only defined when one kernel runs at a time (LT_FLAG_SERIAL / stats launches)
   const bool timeKinds = timeTrace && plan.streams == 1;
   const LtSceneDev sc = scene_for_plan(scene, plan);
+  LtViews views = {viewCount, cams, nullptr};
+  if (wavefront && viewCount > 1) {  // the frameCount of every (view, frame) pair, for the shade kernels
+    const size_t n = (size_t)viewCount * L.frames;
+    std::vector<unsigned> fc(n);
+    for (int v = 0; v < viewCount; v++)
+      for (int f = 0; f < L.frames; f++) fc[(size_t)v * L.frames + f] = cams[v].frameCount + (unsigned)f * L.frameStride;
+    if (ctx->viewFrameCountsSize < n) {
+      if (ctx->dViewFrameCounts) cudaFree(ctx->dViewFrameCounts);
+      ctx->dViewFrameCounts = nullptr;
+      ctx->viewFrameCountsSize = 0;
+      CK(cudaMalloc(&ctx->dViewFrameCounts, n * sizeof(unsigned)));
+      ctx->viewFrameCountsSize = n;
+    }
+    // pageable source: staged before the call returns, so fc may go
+    CK(cudaMemcpyAsync(ctx->dViewFrameCounts, fc.data(), n * sizeof(unsigned), cudaMemcpyHostToDevice, ctx->stream));
+    views.dFrameCounts = ctx->dViewFrameCounts;
+  }
   CK(cudaEventRecord(ctx->ev0, ctx->stream));
-  int launches = wavefront ? lt_launch_render_wavefront(sc, plan, L, dOut, ctx->dCounters, ctx->wfWorkspace,
-                                                        ctx->stats.sm_count, ctx->stream,
-                                                        timeTrace ? ctx->traceEvents.data() : nullptr, kMaxTracePairs,
-                                                        &tracePairs, timeKinds ? ctx->pairKinds.data() : nullptr,
-                                                        &ctx->wfAux)
-                           : lt_launch_render(sc, plan, L, dOut, ctx->dCounters, ctx->dWork, ctx->stream);
+  int launches = 0;
+  if (wavefront) {
+    launches = lt_launch_render_wavefront(sc, plan, L, dOut, ctx->dCounters, ctx->wfWorkspace, ctx->stats.sm_count,
+                                          ctx->stream, timeTrace ? ctx->traceEvents.data() : nullptr, kMaxTracePairs,
+                                          &tracePairs, timeKinds ? ctx->pairKinds.data() : nullptr, &ctx->wfAux,
+                                          viewCount > 1 ? &views : nullptr);
+  } else if (viewCount > 1) {  // the megakernels: one launch per view, back to back on the stream
+    for (int v = 0; v < viewCount; v++) {
+      LtLaunch Lv = L;
+      Lv.cam = cams[v];
+      launches += lt_launch_render(sc, plan, Lv, dOut + (size_t)v * L.width * L.height * L.depth, ctx->dCounters,
+                                   ctx->dWork, ctx->stream);
+    }
+  } else {
+    launches = lt_launch_render(sc, plan, L, dOut, ctx->dCounters, ctx->dWork, ctx->stream);
+  }
   CK(cudaGetLastError());
   CK(cudaEventRecord(ctx->ev1, ctx->stream));
   ctx->stats.kernel_launches = launches;
@@ -1569,7 +1626,7 @@ static int render_common(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, float*
     CK(cudaStreamSynchronize(ctx->stream));
     CK(cudaEventElapsedTime(&ctx->stats.kernel_ms, ctx->ev0, ctx->ev1));
     ctx->stats.trace_ms = wavefront ? 0.0f : ctx->stats.kernel_ms;
-    ctx->stats.trace_launches = wavefront ? 0 : 1;
+    ctx->stats.trace_launches = wavefront ? 0 : launches;
     ctx->stats.shade_ms = ctx->stats.primary_shade_ms = ctx->stats.accumulate_ms = 0.0f;
     ctx->stats.shade_launches = 0;
     for (int i = 0; i < tracePairs; i++) {
@@ -1717,6 +1774,68 @@ extern "C" int lt_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, con
   if (rc != LT_OK) return rc;
   if (host_out) return download(ctx, host_out, ctx->dOut, floats * sizeof(float));
   return LT_OK;
+}
+
+// the cameras of a views call, with its argument checks (before any device is touched)
+static int check_views(lt_ctx* ctx, const void* cameras28, int view_count, const char* who,
+                       std::vector<RefCamera>* cams) {
+  const std::string w = std::string(who) + ": ";
+  if (view_count < 1) return fail(ctx, LT_ERR_INVALID, w + "view_count must be >= 1");
+  if (!cameras28) return fail(ctx, LT_ERR_INVALID, w + "cameras28 is NULL");
+  if (!ctx) return fail(nullptr, LT_ERR_INVALID, w + "ctx is NULL");
+  cams->resize((size_t)view_count);
+  memcpy(cams->data(), cameras28, sizeof(RefCamera) * (size_t)view_count);
+  return LT_OK;
+}
+
+int lt_internal_render_views(lt_ctx* ctx, lt_scene* scene, const RefCamera* cams, int count,
+                             const lt_render_params* params, float* host_out, int hostFirst, int hostStride) {
+  LtLaunch L;
+  int rc = check_params(ctx, scene, cams, params, &L);
+  if (rc != LT_OK) return rc;
+  CK(cudaSetDevice(ctx->device));
+  const size_t image = (size_t)L.width * L.height * L.depth, floats = image * (size_t)count;
+  if (ctx->viewsFloats < floats) {
+    if (ctx->dViews) cudaFree(ctx->dViews);
+    ctx->dViews = nullptr;
+    ctx->viewsFloats = 0;
+    CK(cudaMalloc(&ctx->dViews, floats * sizeof(float)));
+    ctx->viewsFloats = floats;
+  }
+  // every view accumulates from zero, as after lt_accum_reset
+  CK(cudaMemsetAsync(ctx->dViews, 0, floats * sizeof(float), ctx->stream));
+  rc = render_common(ctx, scene, L, ctx->dViews, true, cams, count);
+  if (rc != LT_OK || !host_out) return rc;
+  if (hostStride == 1) return download(ctx, host_out + (size_t)hostFirst * image, ctx->dViews, floats * sizeof(float));
+  for (int k = 0; k < count && rc == LT_OK; k++)
+    rc = download(ctx, host_out + (size_t)(hostFirst + (size_t)k * hostStride) * image, ctx->dViews + (size_t)k * image,
+                  image * sizeof(float));
+  return rc;
+}
+
+extern "C" int lt_render_views(lt_ctx* ctx, lt_scene* scene, const void* cameras28, int view_count,
+                               const lt_render_params* params, float* host_out) {
+  std::vector<RefCamera> cams;
+  if (int rc = check_views(ctx, cameras28, view_count, "lt_render_views", &cams)) return rc;
+  if (ctx->group) {
+    if (view_count == 1) return lt_multi_render(ctx, scene, cameras28, params, host_out, nullptr);
+    return lt_multi_render_views(ctx, scene, cams.data(), view_count, params, host_out);
+  }
+  return lt_internal_render_views(ctx, scene, cams.data(), view_count, params, host_out, 0, 1);
+}
+
+extern "C" int lt_render_views_device(lt_ctx* ctx, lt_scene* scene, const void* cameras28, int view_count,
+                                      const lt_render_params* params, float* device_out, int sync) {
+  std::vector<RefCamera> cams;
+  if (int rc = check_views(ctx, cameras28, view_count, "lt_render_views_device", &cams)) return rc;
+  if (ctx->group)
+    return fail(ctx, LT_ERR_UNSUPPORTED,
+                "lt_render_views_device: a multi-GPU context renders into host memory (lt_render_views)");
+  LtLaunch L;
+  int rc = check_params(ctx, scene, cameras28, params, &L);
+  if (rc != LT_OK) return rc;
+  if (!device_out) return fail(ctx, LT_ERR_INVALID, "lt_render_views_device: device_out is NULL");
+  return render_common(ctx, scene, L, device_out, sync != 0, cams.data(), view_count);
 }
 
 extern "C" int lt_plugin_load(lt_ctx* ctx, const char* kernel_file_path, int* out_plugin_id) {

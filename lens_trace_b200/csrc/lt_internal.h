@@ -55,7 +55,7 @@ int lt_launch_primary_hits(const LtSceneDev& sc, const LtPlan& plan, const RefCa
 // Dynamic shared memory beyond 48 KB needs an opt-in per kernel and device: given once for every traversal kernel
 // (both files), the first time a launch asks for more.
 void lt_opt_in_traversal_smem(size_t smem);
-extern const void* const lt_wf_traversal_kernels[5];  // lt_wavefront.cu
+extern const void* const lt_wf_traversal_kernels[7];  // lt_wavefront.cu
 int lt_launch_debug_random(const float* fx, const float* fy, const float* seed, int n, float* out, cudaStream_t stream);
 int lt_launch_debug_hemisphere(const float* u1, const float* u2, const float* up, int n, float* out,
                                cudaStream_t stream);
@@ -63,6 +63,16 @@ int lt_launch_debug_hemisphere(const float* u1, const float* u2, const float* up
 // wavefront pipeline (lt_wavefront.cu)
 size_t lt_wf_workspace_bytes_padded(long long nPaths);
 size_t lt_wf_primary_hits_bytes(long long pixels);  // per-launch primary hit records, kept behind the batch workspaces
+// a call of several views: views a batch of batchFrames (view, frame) pairs touches at most, and the primary records of
+// that many views, kept per batch workspace instead of the launch's one set
+int lt_wf_views_per_batch(int batchFrames, int frames, int views);
+size_t lt_wf_view_records_bytes(long long pixels, int viewsPerBatch);
+// The views of one lt_render_views call on one device: view v renders camera cams[v] into dOut + v * W * H * depth.
+struct LtViews {
+  int count;
+  const RefCamera* cams;         // host memory
+  const unsigned* dFrameCounts;  // device memory: frameCount of each (view, frame) pair, view-major (count * frames)
+};
 // traceEvents: optional pool of 2*maxTraceLaunches events; when given, every traversal launch is bracketed by a
 // pair of events and *traceLaunches receives the number of pairs recorded
 // aux: a second stream + events (fork, one batch-order event per stream), used when the plan overlaps consecutive
@@ -79,7 +89,7 @@ enum { LT_TIMED_TRAVERSAL = 0, LT_TIMED_SHADE = 1, LT_TIMED_PRIMARY_SHADE = 2, L
 int lt_launch_render_wavefront(const LtSceneDev& sc, const LtPlan& plan, const LtLaunch& L, float* dOut,
                                LtCounters* dCounters, void* workspace, int smCount, cudaStream_t stream,
                                cudaEvent_t* traceEvents, int maxTraceLaunches, int* traceLaunches,
-                               unsigned char* pairKinds, const LtWfAux* aux);
+                               unsigned char* pairKinds, const LtWfAux* aux, const LtViews* views);
 
 // user-written CUDA kernels with the reference's plug-in ABI (lt_plugin.cu)
 #include <string>
@@ -151,6 +161,10 @@ struct lt_ctx {
   void* wfWorkspace = nullptr;  // wavefront path state / ray queues (two batch workspaces when batches overlap)
   size_t wfBytes = 0;
   LtWfAux wfAux = {};           // second stream + events for overlapping consecutive wavefront batches
+  float* dViews = nullptr;      // the images of an lt_render_views call (not the accumulator dOut)
+  size_t viewsFloats = 0;
+  unsigned* dViewFrameCounts = nullptr;  // LtViews::dFrameCounts of a wavefront views launch
+  size_t viewFrameCountsSize = 0;
   size_t totalMem = 0;
   char* stage = nullptr;  // pinned staging buffer of lt_render's copy into a pageable destination
   size_t stageBytes = 0;
@@ -195,6 +209,12 @@ int lt_internal_download(lt_ctx* ctx, float* host_out, const float* dSrc, size_t
 // one device's share of a render call: like lt_render_device, with the row window of a tile split
 int lt_internal_render_rows(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params,
                             float* device_out, int fullHeight, int rowBlock, int rowStride, int rowPhase, int sync);
+// lt_render_views on one device: view k (camera cams[k]) into the context's view buffer, from zero, and then (host_out
+// != NULL) to host_out + (hostFirst + k * hostStride) * W * H * depth
+int lt_internal_render_views(lt_ctx* ctx, lt_scene* scene, const RefCamera* cams, int count,
+                             const lt_render_params* params, float* host_out, int hostFirst, int hostStride);
+int lt_multi_render_views(lt_ctx* ctx, lt_scene* scene, const RefCamera* cams, int count, const lt_render_params* params,
+                          float* host_out);
 // params->frames frames of a plug-in into ctx->dOut, combined by params->accum_mode (arguments already checked); `who`
 // names the entry point in error messages
 int lt_internal_render_plugin(lt_ctx* ctx, lt_scene* scene, const RefCamera& cam, const lt_render_params& P,

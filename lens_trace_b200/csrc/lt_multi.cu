@@ -521,3 +521,46 @@ int lt_multi_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt
   cudaSetDevice(g->ctx[0]->device);
   return LT_OK;
 }
+
+// Views of one call: device k renders views k, k + G, ... with the single-GPU path and copies each into its place in
+// host_out.  Views are independent, so no collective is involved.
+int lt_multi_render_views(lt_ctx* ctx, lt_scene* scene, const RefCamera* cams, int count, const lt_render_params* params,
+                          float* host_out) {
+  LtGroup* g = ctx->group;
+  const std::string who = "lt_render_views: ";
+  if (!scene || !params) return lt_internal_fail(ctx, LT_ERR_INVALID, who + "NULL argument");
+  if (scene->parts.size() != g->ctx.size())
+    return lt_internal_fail(ctx, LT_ERR_INVALID, who + "the scene was not uploaded through this multi-GPU context");
+  if (params->struct_size != sizeof(lt_render_params) && params->struct_size != offsetof(lt_render_params, split_mode))
+    return lt_internal_fail(ctx, LT_ERR_INVALID, who + "params.struct_size mismatch");
+  lt_render_params P;
+  memset(&P, 0, sizeof P);
+  memcpy(&P, params, params->struct_size < sizeof P ? params->struct_size : sizeof P);
+  P.struct_size = sizeof P;
+  if (P.split_mode != LT_SPLIT_AUTO)
+    return lt_internal_fail(ctx, LT_ERR_INVALID, who + "views are dealt to the devices whole: split_mode must be LT_SPLIT_AUTO");
+  if (P.flags & LT_FLAG_STATS)
+    return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED, who + "LT_FLAG_STATS counts on a single-GPU context");
+  const int G = (int)g->ctx.size();
+  std::vector<int> rcs(G, LT_OK);
+  std::vector<std::thread> workers;
+  for (int k = 0; k < G && k < count; k++)
+    workers.emplace_back([&, k]() {
+      std::vector<RefCamera> mine;
+      for (int v = k; v < count; v += G) mine.push_back(cams[v]);
+      rcs[k] = lt_internal_render_views(g->ctx[k], scene->parts[k], mine.data(), (int)mine.size(), &P, host_out, k, G);
+    });
+  for (std::thread& t : workers) t.join();
+  for (int k = 0; k < G; k++)
+    if (rcs[k] != LT_OK) return lt_internal_fail(ctx, rcs[k], lt_last_error(g->ctx[k]));
+  // statistics of the call: the slowest device's kernels, all devices' launches
+  ctx->stats.kernel_ms = 0.0f;
+  ctx->stats.kernel_launches = 0;
+  for (int k = 0; k < G && k < count; k++) {
+    const lt_ctx* c = g->ctx[k];
+    if (c->stats.kernel_ms > ctx->stats.kernel_ms) ctx->stats.kernel_ms = c->stats.kernel_ms;
+    ctx->stats.kernel_launches += c->stats.kernel_launches;
+  }
+  cudaSetDevice(g->ctx[0]->device);
+  return LT_OK;
+}

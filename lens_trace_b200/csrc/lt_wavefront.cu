@@ -191,9 +191,12 @@ __device__ __forceinline__ void queue_append_warp(const LtWfBuffers& B, int dst,
   }
 }
 
-__device__ __forceinline__ unsigned sample_index_of(const LtLaunch& L, const PathConsts& pc, int frame, int sample) {
-  unsigned fc = L.cam.frameCount + (unsigned)frame * L.frameStride;
+// sample index of a path whose frame has camera frameCount fc
+__device__ __forceinline__ unsigned sample_index_fc(const PathConsts& pc, unsigned fc, int sample) {
   return pc.samplesPerFrame == 25 ? fc * 32u + (unsigned)sample : fc;
+}
+__device__ __forceinline__ unsigned sample_index_of(const LtLaunch& L, const PathConsts& pc, int frame, int sample) {
+  return sample_index_fc(pc, L.cam.frameCount + (unsigned)frame * L.frameStride, sample);
 }
 
 // Round 0 fused: camera ray -> trace -> shade for every path of the batch.  Primary rays are coherent
@@ -214,6 +217,9 @@ struct LtWfPrimary {
   int* alive;          // compacted list of alive pixels
   unsigned char* cls;  // per pixel: 0 black, 1 white, 2 alive
   int* aliveCount;
+  // a call of several views (lt_render_views): frameCount of each (view, frame) pair of the batch, in batch order;
+  // nullptr otherwise (the frames of the one camera L.cam)
+  const unsigned* frameCounts;
 };
 
 __device__ __forceinline__ void film_of_path(const LtWfPrimary& P, long long path, int pixels, const LtLaunch& L,
@@ -269,10 +275,12 @@ __global__ void __launch_bounds__(WF_BLOCK) k_wf_primary_trace(LtSceneDev sc, Lt
 // P.alive != nullptr: only the alive pixels get paths (nf frames x aliveCount pixels, enumerated through the list);
 // the path id stays frame * pixels + pixel, so nothing downstream changes.
 // out: the kind of round 1 (WF_FIRST_SHADOW, or WF_GENERIC), which decides what its entries hold
-template <bool STATS>
+// VIEWS: the nf frames are one view's frames inside a batch that holds several views (L.cam is that view's camera, P
+// its records); their paths are numbered from pathBase in the batch
+template <bool STATS, bool VIEWS>
 __global__ void __launch_bounds__(WF_BLOCK) k_wf_primary(LtSceneDev sc, LtLaunch L, LtWfBuffers B, int nf,
                                                          int pixels, int sample, LtCounters* gcnt, LtWfPrimary P,
-                                                         int out) {
+                                                         int out, int pathBase) {
   LT_TRAV_SMEM(s, lt_stack_levels(sc))
   const float4* __restrict__ primaryHits = P.hits;
   const bool cull = (L.flags & LT_DEV_FLAG_CULL) != 0;  // closest-hit rays skip subtrees behind the current hit
@@ -322,6 +330,7 @@ __global__ void __launch_bounds__(WF_BLOCK) k_wf_primary(LtSceneDev sc, LtLaunch
       path_reset(ps);
       const Hit h = t.h;
       bool done = shade_step(sc, pc, ps, t.r, h, fx, fy, sample_index_of(L, pc, fl, sample), tStart, ignore, anyHit);
+      if (VIEWS) p += pathBase;
       if (done) {
         float col[3], fc[3] = {0.0f, 0.0f, 0.0f};
         sample_colour(pc, ps, col);
@@ -443,8 +452,8 @@ __global__ void __launch_bounds__(WF_BLOCK) __maxnreg__(STATS ? 64 : 56)
 // K (WfRound) is the kind of the round: it fixes the stage of every entry and which arrays are loaded.  A shadow
 // result reads ray, hit word, payA and (after the first bounce) payB / payC; an extension result reads neither its ray
 // nor the normal: a surface hit rebuilds the shading point from the hit, a light hit reads dLight, a miss only
-// finishes the sample.
-template <int Q, int K>
+// finishes the sample.  VIEWS: the batch holds (view, frame) pairs; P.frameCounts gives each pair's frameCount.
+template <int Q, int K, bool VIEWS>
 __global__ void __launch_bounds__(WF_BLOCK, 8) k_wf_shade(LtSceneDev sc, LtLaunch L, LtWfBuffers B, int pixels,
                                                           int frame0, int sample, LtWfPrimary P) {
   constexpr int q = Q;
@@ -512,7 +521,8 @@ __global__ void __launch_bounds__(WF_BLOCK, 8) k_wf_shade(LtSceneDev sc, LtLaunc
       int fl;
       float fx, fy;
       film_of_path(P, path, pixels, L, fl, fx, fy);
-      unsigned sampleIndex = sample_index_of(L, pc, frame0 + fl, sample);
+      unsigned sampleIndex =
+          VIEWS ? sample_index_fc(pc, P.frameCounts[fl], sample) : sample_index_of(L, pc, frame0 + fl, sample);
       bool done = shade_step(sc, pc, ps, r, h, fx, fy, sampleIndex, tStart, ignore, anyHit, lightHit ? 1 : 0);
       if (done) {
         float col[3], fc[3] = {0.0f, 0.0f, 0.0f};
@@ -612,10 +622,23 @@ size_t lt_wf_primary_hits_bytes(long long pixels) {
   return (sizeof(float4) + sizeof(float2) + sizeof(int) + 1) * (size_t)pixels + 1024 + 5 * 256;  // 5 arrays, 256-aligned
 }
 
+// Views a batch of batchFrames (view, frame) pairs touches at most: a batch that starts at the last frame of a view
+// reaches (frames + batchFrames - 2) / frames views beyond it.
+int lt_wf_views_per_batch(int batchFrames, int frames, int views) {
+  const long long n = ((long long)frames + batchFrames - 2) / frames + 1;
+  return n < views ? (int)n : views;
+}
+
+// a call of several views keeps, per batch workspace, the primary records of every view its batch touches
+size_t lt_wf_view_records_bytes(long long pixels, int viewsPerBatch) {
+  return ((lt_wf_primary_hits_bytes(pixels) + 255) & ~(size_t)255) * (size_t)viewsPerBatch;
+}
+
 // the kernels whose shared memory grows with the stack depth (lt_opt_in_traversal_smem)
-const void* const lt_wf_traversal_kernels[5] = {
-    (const void*)k_wf_primary_trace, (const void*)k_wf_primary<false>, (const void*)k_wf_primary<true>,
-    (const void*)k_wf_trace<false, false>, (const void*)k_wf_trace<true, false>};
+const void* const lt_wf_traversal_kernels[7] = {
+    (const void*)k_wf_primary_trace,      (const void*)k_wf_primary<false, false>, (const void*)k_wf_primary<true, false>,
+    (const void*)k_wf_primary<false, true>, (const void*)k_wf_primary<true, true>,   (const void*)k_wf_trace<false, false>,
+    (const void*)k_wf_trace<true, false>};
 
 // Round r >= 1 of a sample (WfRound).  The exact pipelines fold the retracing of a light hit into its shading, so round
 // 1 holds the first shadow rays of the paths, and after it extension and shadow rounds alternate: an extension result
@@ -626,21 +649,41 @@ static int wf_round_kind(int flags, int r) {
   return r == 1 ? WF_FIRST_SHADOW : (r & 1) ? WF_SHADOW : WF_EXTENSION;
 }
 
-template <int Q>
+template <int Q, bool V>
 static void launch_shade(int kind, int grid, cudaStream_t st, const LtSceneDev& sc, const LtLaunch& L,
                          const LtWfBuffers& B, int pixels, int sample, const LtWfPrimary& P) {
   switch (kind) {
-    case WF_FIRST_SHADOW: k_wf_shade<Q, WF_FIRST_SHADOW><<<grid, WF_BLOCK, 0, st>>>(sc, L, B, pixels, 0, sample, P); break;
-    case WF_SHADOW: k_wf_shade<Q, WF_SHADOW><<<grid, WF_BLOCK, 0, st>>>(sc, L, B, pixels, 0, sample, P); break;
-    case WF_EXTENSION: k_wf_shade<Q, WF_EXTENSION><<<grid, WF_BLOCK, 0, st>>>(sc, L, B, pixels, 0, sample, P); break;
-    default: k_wf_shade<Q, WF_GENERIC><<<grid, WF_BLOCK, 0, st>>>(sc, L, B, pixels, 0, sample, P); break;
+    case WF_FIRST_SHADOW: k_wf_shade<Q, WF_FIRST_SHADOW, V><<<grid, WF_BLOCK, 0, st>>>(sc, L, B, pixels, 0, sample, P); break;
+    case WF_SHADOW: k_wf_shade<Q, WF_SHADOW, V><<<grid, WF_BLOCK, 0, st>>>(sc, L, B, pixels, 0, sample, P); break;
+    case WF_EXTENSION: k_wf_shade<Q, WF_EXTENSION, V><<<grid, WF_BLOCK, 0, st>>>(sc, L, B, pixels, 0, sample, P); break;
+    default: k_wf_shade<Q, WF_GENERIC, V><<<grid, WF_BLOCK, 0, st>>>(sc, L, B, pixels, 0, sample, P); break;
   }
+}
+
+// The views of a batch: one segment per view it touches, (view, frames first .. first + count - 1 of that view) at pair
+// offset `at` of the batch.  Pairs are view-major, so the segments of a batch are consecutive views.
+struct WfSegment {
+  int view, first, count, at;
+};
+static int batch_segments(long long pair0, int nf, int frames, WfSegment* seg) {
+  int n = 0;
+  for (int at = 0; at < nf;) {
+    const long long pair = pair0 + at;
+    WfSegment s;
+    s.view = (int)(pair / frames);
+    s.first = (int)(pair - (long long)s.view * frames);
+    s.count = frames - s.first < nf - at ? frames - s.first : nf - at;
+    s.at = at;
+    seg[n++] = s;
+    at += s.count;
+  }
+  return n;
 }
 
 int lt_launch_render_wavefront(const LtSceneDev& sc, const LtPlan& plan, const LtLaunch& L, float* dOut,
                                LtCounters* dCounters, void* workspace, int smCount, cudaStream_t stream,
                                cudaEvent_t* traceEvents, int maxTraceLaunches, int* traceLaunches,
-                               unsigned char* pairKinds, const LtWfAux* aux) {
+                               unsigned char* pairKinds, const LtWfAux* aux, const LtViews* views) {
   int pairs = 0;
   // which: 0 = before, 1 = after a launch; kind (LT_TIMED_*): what the bracketed kernel does.  Traversal launches
   // are always bracketed when events are given, the other kinds only when the caller passes pairKinds.
@@ -659,11 +702,22 @@ int lt_launch_render_wavefront(const LtSceneDev& sc, const LtPlan& plan, const L
   const int batchFrames = plan.batchFrames;
   const size_t smem = plan.smemStack;
   const size_t wsBytes = lt_wf_workspace_bytes_padded((long long)batchFrames * pixels);
+  // A call of several views: the batches run over (view, frame) pairs, view-major, so every view's frames still reach
+  // its image in frame order.  Each batch traces the camera rays of the views it touches into its own record slots
+  // (one per view, behind the batch workspaces); a view whose frames two batches share is traced by both, to the same
+  // records.
+  const int V = views ? views->count : 1;
+  const long long totalPairs = (long long)L.frames * V;
+  const int viewsPerBatch = views ? lt_wf_views_per_batch(batchFrames, L.frames, V) : 1;
+  const size_t slotBytes = (lt_wf_primary_hits_bytes(pixels) + 255) & ~(size_t)255;
+  const size_t imageFloats = (size_t)pixels * L.depth;
   int preLaunches = 0;
-  // primary hits once per pixel per launch; kept behind the batch workspaces
-  LtWfPrimary P = {};
-  if (plan.sharedPrimary) {
-    char* pb = (char*)workspace + (size_t)plan.streams * wsBytes;  // 256-aligned: wsBytes is a multiple of 256
+  int l = 0;
+  while ((1ll << l) < pixels) l++;
+  // the primary records of slot k of side `side` (one launch: slot 0 of side 0)
+  auto records = [&](int side, int k) {
+    LtWfPrimary P = {};
+    char* pb = (char*)workspace + (size_t)plan.streams * wsBytes + ((size_t)side * viewsPerBatch + k) * slotBytes;
     auto take = [&](size_t bytes) {
       char* r = pb;
       pb += (bytes + 255) & ~(size_t)255;
@@ -671,48 +725,93 @@ int lt_launch_render_wavefront(const LtSceneDev& sc, const LtPlan& plan, const L
     };
     P.hits = (float4*)take(sizeof(float4) * (size_t)pixels);
     P.film = (float2*)take(sizeof(float2) * (size_t)pixels);
-    int l = 0;
-    while ((1ll << l) < pixels) l++;
     P.divS = 25 + l;
     P.divM = (unsigned long long)(((1ull << P.divS) + (unsigned long long)pixels - 1ull) / (unsigned long long)pixels);
     if (plan.classify) {
       P.alive = (int*)take(sizeof(int) * (size_t)pixels);
       P.aliveCount = (int*)take(256);
       P.cls = (unsigned char*)take((size_t)pixels);
-      cudaMemsetAsync(P.aliveCount, 0, sizeof(int), stream);
     }
-    mark(0, stream);
-    k_wf_primary_trace<<<(pixels + WF_BLOCK - 1) / WF_BLOCK, WF_BLOCK, smem, stream>>>(sc, L, P, pixels,
-                                                                                         plan.classify ? 1 : 0);
-    mark(1, stream);
+    return P;
+  };
+  auto trace_primary = [&](const LtLaunch& Lv, const LtWfPrimary& P, cudaStream_t st) {
+    if (plan.classify) cudaMemsetAsync(P.aliveCount, 0, sizeof(int), st);
+    mark(0, st);
+    k_wf_primary_trace<<<(pixels + WF_BLOCK - 1) / WF_BLOCK, WF_BLOCK, smem, st>>>(sc, Lv, P, pixels,
+                                                                                  plan.classify ? 1 : 0);
+    mark(1, st);
+  };
+  // primary hits once per pixel per launch; kept behind the batch workspaces
+  LtWfPrimary P = {};
+  if (plan.sharedPrimary && !views) {
+    P = records(0, 0);
+    trace_primary(L, P, stream);
     preLaunches = 1;
   }
-  float4* primaryHits = P.hits;
   if (overlap) {
     cudaEventRecord(aux->fork, stream);
     cudaStreamWaitEvent(aux->extra, aux->fork, 0);
   }
+  std::vector<WfSegment> segs((size_t)viewsPerBatch);
+  std::vector<LtWfPrimary> segP((size_t)viewsPerBatch);
+  std::vector<LtLaunch> segL((size_t)viewsPerBatch);
   int launches = preLaunches, batch = 0, lastSide = 0;
-  for (int frame0 = 0; frame0 < L.frames; frame0 += batchFrames, batch++) {
+  for (long long pair0 = 0; pair0 < totalPairs; pair0 += batchFrames, batch++) {
     const int side = overlap ? (batch & 1) : 0;
     cudaStream_t st = side ? aux->extra : stream;
-    int nf = L.frames - frame0 < batchFrames ? L.frames - frame0 : batchFrames;
+    int nf = totalPairs - pair0 < batchFrames ? (int)(totalPairs - pair0) : batchFrames;
     long long nPaths = (long long)nf * pixels;
     LtWfBuffers B = carve((char*)workspace + (size_t)side * wsBytes, (long long)batchFrames * pixels);
     LtLaunch Lb = L;
-    Lb.cam.frameCount = L.cam.frameCount + (unsigned)frame0 * L.frameStride;  // frame index 0 of the batch
+    int nSeg = 0;
+    if (views) {
+      nSeg = batch_segments(pair0, nf, L.frames, segs.data());
+      for (int k = 0; k < nSeg; k++) {
+        segL[k] = L;
+        segL[k].cam = views->cams[segs[k].view];
+        segP[k] = plan.sharedPrimary ? records(side, k) : LtWfPrimary{};
+        if (plan.sharedPrimary) {
+          trace_primary(segL[k], segP[k], st);
+          launches++;
+        }
+      }
+      // the shade kernels take the film table of the first slot (it does not depend on the camera) and each pair's
+      // frameCount
+      P = segP[0];
+      P.frameCounts = views->dFrameCounts + pair0;
+    } else {
+      Lb.cam.frameCount = L.cam.frameCount + (unsigned)pair0 * L.frameStride;  // frame index 0 of the batch
+    }
     int grid = (int)((nPaths + WF_BLOCK - 1) / WF_BLOCK);
     if (grid > smCount * 32) grid = smCount * 32;
     for (int s = 0; s < plan.samplesPerFrame; s++) {
       // round 0 (primary rays) fused into one kernel; its survivors are queue 0
       k_wf_reset<<<1, 1, 0, st>>>(B);
-      // a traversal kernel only when it traces the camera rays itself
-      mark(0, st, primaryHits ? LT_TIMED_PRIMARY_SHADE : LT_TIMED_TRAVERSAL);
       const int out = wf_round_kind(L.flags, 1);
-      if (stats) k_wf_primary<true><<<grid, WF_BLOCK, smem, st>>>(sc, Lb, B, nf, pixels, s, dCounters, P, out);
-      else k_wf_primary<false><<<grid, WF_BLOCK, smem, st>>>(sc, Lb, B, nf, pixels, s, nullptr, P, out);
-      mark(1, st, primaryHits ? LT_TIMED_PRIMARY_SHADE : LT_TIMED_TRAVERSAL);
-      launches += 2;
+      if (views) {  // one launch per view of the batch, its paths numbered from its pair offset
+        for (int k = 0; k < nSeg; k++) {
+          LtLaunch Ls = segL[k];
+          Ls.cam.frameCount = segL[k].cam.frameCount + (unsigned)segs[k].first * L.frameStride;
+          int g = (int)(((long long)segs[k].count * pixels + WF_BLOCK - 1) / WF_BLOCK);
+          if (g > smCount * 32) g = smCount * 32;
+          mark(0, st, plan.sharedPrimary ? LT_TIMED_PRIMARY_SHADE : LT_TIMED_TRAVERSAL);
+          if (stats)
+            k_wf_primary<true, true><<<g, WF_BLOCK, smem, st>>>(sc, Ls, B, segs[k].count, pixels, s, dCounters,
+                                                                segP[k], out, segs[k].at * pixels);
+          else
+            k_wf_primary<false, true><<<g, WF_BLOCK, smem, st>>>(sc, Ls, B, segs[k].count, pixels, s, nullptr,
+                                                                 segP[k], out, segs[k].at * pixels);
+          mark(1, st, plan.sharedPrimary ? LT_TIMED_PRIMARY_SHADE : LT_TIMED_TRAVERSAL);
+        }
+        launches += 1 + nSeg;
+      } else {
+        // a traversal kernel only when it traces the camera rays itself
+        mark(0, st, plan.sharedPrimary ? LT_TIMED_PRIMARY_SHADE : LT_TIMED_TRAVERSAL);
+        if (stats) k_wf_primary<true, false><<<grid, WF_BLOCK, smem, st>>>(sc, Lb, B, nf, pixels, s, dCounters, P, out, 0);
+        else k_wf_primary<false, false><<<grid, WF_BLOCK, smem, st>>>(sc, Lb, B, nf, pixels, s, nullptr, P, out, 0);
+        mark(1, st, plan.sharedPrimary ? LT_TIMED_PRIMARY_SHADE : LT_TIMED_TRAVERSAL);
+        launches += 2;
+      }
       int q = 0;
       for (int r = 1; r < plan.rounds; r++) {
         const int kind = wf_round_kind(L.flags, r);
@@ -723,8 +822,13 @@ int lt_launch_render_wavefront(const LtSceneDev& sc, const LtPlan& plan, const L
         else k_wf_trace<false, false><<<plan.grid, WF_BLOCK, smem, st>>>(sc, Lb, B, q, nullptr, B.rayO[q], B.rayD[q], hitWords);
         mark(1, st);
         mark(0, st, LT_TIMED_SHADE);
-        if (q == 0) launch_shade<0>(kind, grid, st, sc, Lb, B, pixels, s, P);
-        else launch_shade<1>(kind, grid, st, sc, Lb, B, pixels, s, P);
+        if (views) {
+          if (q == 0) launch_shade<0, true>(kind, grid, st, sc, Lb, B, pixels, s, P);
+          else launch_shade<1, true>(kind, grid, st, sc, Lb, B, pixels, s, P);
+        } else {
+          if (q == 0) launch_shade<0, false>(kind, grid, st, sc, Lb, B, pixels, s, P);
+          else launch_shade<1, false>(kind, grid, st, sc, Lb, B, pixels, s, P);
+        }
         mark(1, st, LT_TIMED_SHADE);
         k_wf_swap<<<1, 1, 0, st>>>(B, q);
         launches += 3;
@@ -734,11 +838,21 @@ int lt_launch_render_wavefront(const LtSceneDev& sc, const LtPlan& plan, const L
     // the frame combiner is applied in frame order: this batch's accumulate follows the previous batch's
     if (overlap && batch > 0) cudaStreamWaitEvent(st, aux->order[1 - side], 0);
     mark(0, st, LT_TIMED_ACCUMULATE);
-    k_wf_accumulate<<<(pixels + WF_BLOCK - 1) / WF_BLOCK, WF_BLOCK, 0, st>>>(L, B, dOut, pixels, frame0, nf, P.cls);
+    if (views) {  // each view's frames of the batch into its own image
+      for (int k = 0; k < nSeg; k++) {
+        LtWfBuffers Bs = B;
+        Bs.frameCol = B.frameCol + (size_t)segs[k].at * pixels;
+        k_wf_accumulate<<<(pixels + WF_BLOCK - 1) / WF_BLOCK, WF_BLOCK, 0, st>>>(
+            segL[k], Bs, dOut + (size_t)segs[k].view * imageFloats, pixels, segs[k].first, segs[k].count, segP[k].cls);
+      }
+      launches += nSeg;
+    } else {
+      k_wf_accumulate<<<(pixels + WF_BLOCK - 1) / WF_BLOCK, WF_BLOCK, 0, st>>>(L, B, dOut, pixels, (int)pair0, nf, P.cls);
+      launches++;
+    }
     mark(1, st, LT_TIMED_ACCUMULATE);
     if (overlap) cudaEventRecord(aux->order[side], st);
     lastSide = side;
-    launches++;
   }
   // join: the last accumulate follows every earlier one (chain of order events), and every stream's last kernel is
   // its accumulate, so waiting for the last batch's event puts all of it before what follows on `stream`

@@ -29,7 +29,7 @@ class RenderExtensionB200(C.Structure):
         ("sType", C.c_int), ("pNext", C.c_void_p), ("frames", C.c_uint32), ("accumulate", C.c_uint32),
         ("maxRayDepth", C.c_uint32), ("collectStats", C.c_uint32), ("rays", C.c_uint64), ("nodeTests", C.c_uint64),
         ("triTests", C.c_uint64), ("kernelMilliseconds", C.c_float), ("deviceCount", C.c_uint32),
-        ("splitMode", C.c_uint32),
+        ("splitMode", C.c_uint32), ("viewCount", C.c_uint32), ("ppViewCameras", C.c_void_p),
     ]
 
 
@@ -186,12 +186,19 @@ class Renderer:
             self.h = None
 
 
-def make_extension(frames=1, accumulate=False, max_ray_depth=0, collect_stats=False, devices=0, split=0):
+def make_extension(frames=1, accumulate=False, max_ray_depth=0, collect_stats=False, devices=0, split=0,
+                   view_cameras=None):
+    """view_cameras: a list of Camera objects rendered in one call (viewCount, ppViewCameras) instead of the camera
+    given to render(); its `out` then holds len(view_cameras) images."""
     e = RenderExtensionB200()
     e.sType = STRUCTURE_TYPE_RENDER_EXTENSION_B200
     e.pNext = None
     e.frames, e.accumulate, e.maxRayDepth, e.collectStats = frames, int(accumulate), max_ray_depth, int(collect_stats)
     e.deviceCount, e.splitMode = devices, split
+    if view_cameras:
+        e._view_array = (C.c_void_p * len(view_cameras))(*[c.h for c in view_cameras])  # kept alive with e
+        e.viewCount = len(view_cameras)
+        e.ppViewCameras = C.cast(e._view_array, C.c_void_p)
     return e
 
 

@@ -12,6 +12,7 @@
 #include <atomic>
 #include <mutex>
 #include <set>
+#include <vector>
 
 // ---- object identity for the device-scene cache (include/lens_trace/api.h) ----
 namespace {
@@ -247,14 +248,37 @@ void RendererB200::renderCommon(const std::string& kernelFilePath, KernelMode ke
     if (ext->collectStats && wantDevices == 1 && plugin < 0) params.flags |= LT_FLAG_STATS;
     params.split_mode = (int)ext->splitMode;
   }
-  uint64_t need = sizeof(float) * imageDimensions[0] * imageDimensions[1] * imageDimensions[2];
+  const uint32_t views = ext && ext->viewCount >= 2 ? ext->viewCount : 1;
+  uint64_t need = sizeof(float) * imageDimensions[0] * imageDimensions[1] * imageDimensions[2] * views;
   if (outputBufferSize < need) {
-    printf("ERROR: output buffer is %llu bytes, image needs %llu\n", (unsigned long long)outputBufferSize,
+    printf("ERROR: output buffer is %llu bytes, %u image(s) need %llu\n", (unsigned long long)outputBufferSize, views,
            (unsigned long long)need);
     return;
   }
+  std::vector<char> viewCameras;  // the views' 28-byte camera records, back to back
+  if (views > 1) {
+    if (plugin >= 0) {
+      printf("ERROR: RenderExtensionB200::viewCount renders the built-in kernels only, not '%s'\n",
+             kernelFilePath.c_str());
+      return;
+    }
+    if (!ext->ppViewCameras) {
+      printf("ERROR: RenderExtensionB200::viewCount is %u but ppViewCameras is NULL\n", views);
+      return;
+    }
+    viewCameras.resize((size_t)views * 28);
+    for (uint32_t v = 0; v < views; v++) {
+      if (!ext->ppViewCameras[v]) {
+        printf("ERROR: RenderExtensionB200::ppViewCameras[%u] is NULL\n", v);
+        return;
+      }
+      memcpy(viewCameras.data() + (size_t)v * 28, ext->ppViewCameras[v]->getCameraBuffer(), 28);
+    }
+  }
   int rc;
-  if (plugin >= 0 && ext)  // frames, accumulation and devices as the extension asks
+  if (views > 1)
+    rc = lt_render_views(useCtx, scene, viewCameras.data(), (int)views, &params, (float*)pOutputBuffer);
+  else if (plugin >= 0 && ext)  // frames, accumulation and devices as the extension asks
     rc = lt_render_plugin_frames(useCtx, scene, camera->getCameraBuffer(), plugin, &params,
                                  isCl && workBlockSize ? (int)workBlockSize[0] : 0,
                                  isCl && workBlockSize ? (int)workBlockSize[1] : 0,
