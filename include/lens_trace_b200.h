@@ -114,7 +114,7 @@ typedef struct lt_stats {
   uint64_t node_tests;  /* boxes tested, reference traversal order */
   uint64_t tri_tests;   /* triangle tests executed, reference traversal order */
   float kernel_ms;      /* device time of the render kernels of the last lt_render* call (CUDA events) */
-  float upload_ms;      /* device time of the last lt_scene_upload (H2D + re-flatten) */
+  float upload_ms;      /* device time of the last lt_scene_upload (H2D + re-flatten) or lt_scene_refit */
   int32_t kernel_launches; /* kernels launched by the last lt_render* call */
   int32_t sm_count;
   float trace_ms;       /* part of kernel_ms spent in the traversal kernels (k_wf_primary + k_wf_trace, or the
@@ -165,6 +165,28 @@ int lt_scene_build_ploc(lt_ctx* ctx, const void* primitives, uint64_t primitive_
                         uint64_t material_bytes, lt_scene** out_scene);
 int lt_scene_download(lt_ctx* ctx, lt_scene* scene, void* nodes, uint64_t node_bytes, void* primitives,
                       uint64_t primitive_bytes, void* light_container);
+/* Replace the primitives of an uploaded scene and refit its tree on the device: moving geometry without a new upload.
+ * primitives: the scene's primitive count of 76-byte Primitive records, in the order of the scene's primitive buffer
+ * (the caller's order for an uploaded scene, the order lt_scene_download returns for a built one).  Materials, the
+ * light container and the topology (child offsets, primitiveCount, axis, the DFS order) stay as they are.
+ * Afterwards every node box is the exact union of its content: a leaf's box covers all primitiveCount triangles from
+ * primitivesOffset, an inner node's box is the union of its two children, with std::min / std::max keeping the first
+ * operand on ties (a triangle's vertices a, b, c in that order, a leaf's primitives in order, the first child before
+ * the second).  The result is deterministic, and every render entry point on the scene then gives byte for byte what
+ * it gives on a scene uploaded with lt_scene_upload from the refitted nodes (lt_scene_download), the new primitives
+ * and the scene's materials and lights.
+ * Rejected with LT_ERR_INVALID, the scene untouched: primitive_bytes other than the primitive count x 76, a
+ * materialIndex out of range, a non-finite vertex coordinate; and a scene with a leaf whose primitiveCount primitives
+ * from primitivesOffset run past its primitive buffer (lt_scene_upload checks only a leaf's first primitive, which
+ * is all the reference's leaves test).  Synchronous: ordered after earlier work on the
+ * context's stream, returns when the scene is ready; lt_stats.upload_ms reports the refit's device time.  On a
+ * multi-GPU context every device's copy is refitted.  After LT_ERR_CUDA the scene is unusable: release it.
+ * A refit keeps the topology: after large deformations a new build (lt_scene_build_ploc) gives a better tree. */
+int lt_scene_refit(lt_ctx* ctx, lt_scene* scene, const void* primitives, uint64_t primitive_bytes);
+/* The same with the primitives in device memory of the context's device (e.g. a torch tensor's data_ptr), checked by
+ * a kernel before anything is overwritten; memory of another device, host memory or a pointer that is not 4-byte
+ * aligned -> LT_ERR_INVALID.  Single-GPU contexts only (LT_ERR_UNSUPPORTED otherwise). */
+int lt_scene_refit_device(lt_ctx* ctx, lt_scene* scene, const void* device_primitives, uint64_t primitive_bytes);
 /* node and primitive counts of a scene */
 int lt_scene_info(const lt_scene* scene, uint64_t* node_count, uint64_t* primitive_count, int32_t* stack_depth);
 
@@ -280,6 +302,9 @@ int lt_debug_traversal_tree(const void* nodes, uint64_t node_bytes, int32_t prim
 /* Test hook: 1 when the pruned threaded copies of an uploaded scene are a traversal tree, 0 when not (also for
  * scenes without host-built copies), < 0 on error. */
 int lt_debug_scene_traversal_tree(const lt_scene* scene);
+/* Test hook: the bytes of device memory a scene holds (all devices' copies of a multi-GPU scene), counted at each
+ * allocation and release the library makes for it. */
+int lt_debug_scene_bytes(const lt_scene* scene, uint64_t* out_bytes);
 
 /* Test hook: full != 0 makes launches on `scene` (single-GPU) walk the full threaded copies for every ray, 0 restores
  * the pruned ones.  The output is the same either way; tests compare the two. */

@@ -21,7 +21,7 @@ SYMBOLS = [
     "lt_debug_gather_peak", "lt_ctx_create_multi", "lt_ctx_device_count", "lt_host_register", "lt_host_unregister", "lt_debug_tile_rows",
     "lt_debug_plan", "lt_debug_ctx_limits", "lt_render_plugin_frames", "lt_debug_build_traversal_tree",
     "lt_debug_scene_traversal_tree", "lt_debug_traversal_tree", "lt_render_views", "lt_render_views_device",
-    "lt_debug_plan_views",
+    "lt_debug_plan_views", "lt_scene_refit", "lt_scene_refit_device", "lt_debug_scene_bytes",
 ]
 
 
@@ -75,6 +75,8 @@ def load():
     lib.lt_scene_build_lbvh.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.POINTER(C.c_void_p)]
     lib.lt_scene_build_ploc.argtypes = lib.lt_scene_build_lbvh.argtypes
     lib.lt_scene_download.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p]
+    lib.lt_scene_refit.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64]
+    lib.lt_scene_refit_device.argtypes = lib.lt_scene_refit.argtypes
     lib.lt_scene_info.argtypes = [C.c_void_p, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_int32)]
     lib.lt_scene_release.argtypes = [C.c_void_p, C.c_void_p]
     lib.lt_scene_release.restype = None
@@ -98,6 +100,7 @@ def load():
     lib.lt_debug_build_traversal_tree.argtypes = [C.c_void_p, C.c_uint64, C.c_int32, C.c_void_p, C.POINTER(C.c_int32),
                                                   C.c_void_p, C.POINTER(C.c_int32)]
     lib.lt_debug_scene_traversal_tree.argtypes = [C.c_void_p]
+    lib.lt_debug_scene_bytes.argtypes = [C.c_void_p, C.POINTER(C.c_uint64)]
     lib.lt_debug_traversal_tree.argtypes = [C.c_void_p, C.c_uint64, C.c_int32, C.c_void_p, C.POINTER(C.c_double)]
     lib.lt_debug_ctx_limits.argtypes = [C.c_void_p, C.c_int, C.c_int]
     lib.lt_debug_plan.argtypes = [C.POINTER(RenderParams), C.c_uint64, C.c_int32, C.c_uint64, C.c_int32,
@@ -231,6 +234,18 @@ class Context:
                                                prims.nbytes, lights.ctypes.data), "lt_scene_download")
         return L.SceneBuffers(nodes, prims, getattr(scene, "materials", np.zeros(0, L.MATERIAL)), lights), sd.value
 
+    def refit(self, scene, prims):
+        """Replace the scene's primitives (layouts.PRIM array in the order of its primitive buffer) and refit its tree
+        on the device (lt_scene_refit); the topology, materials and lights stay."""
+        prims = np.ascontiguousarray(prims, dtype=L.PRIM)
+        self._check(self.lib.lt_scene_refit(self.h, scene.h, prims.ctypes.data, prims.nbytes), "lt_scene_refit")
+
+    def refit_device(self, scene, device_ptr, nbytes):
+        """lt_scene_refit_device: the new primitives are nbytes of device memory at device_ptr (e.g. a torch CUDA
+        tensor's data_ptr())"""
+        self._check(self.lib.lt_scene_refit_device(self.h, scene.h, C.c_void_p(device_ptr), nbytes),
+                    "lt_scene_refit_device")
+
     def render(self, scene, camera, params, want_output=True):
         """Host-buffer path (lt_render): returns float32 [H, W, depth] or None."""
         out = None
@@ -350,6 +365,12 @@ class Context:
         rc = self.lib.lt_debug_scene_traversal_tree(scene.h)
         self._check(min(rc, 0), "lt_debug_scene_traversal_tree")
         return rc == 1
+
+    def scene_bytes(self, scene):
+        """Test hook: the bytes of device memory `scene` holds (lt_debug_scene_bytes)"""
+        out = C.c_uint64(0)
+        self._check(self.lib.lt_debug_scene_bytes(scene.h, C.byref(out)), "lt_debug_scene_bytes")
+        return out.value
 
     def debug_limits(self, threaded_max_nodes, stream_min_nodes):
         """Test hook: trees of at most threaded_max_nodes nodes get host-built threaded copies at upload (larger ones

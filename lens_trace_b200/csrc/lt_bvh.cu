@@ -215,16 +215,28 @@ __global__ void k_karras(const unsigned long long* __restrict__ keys, int n, int
   if (i == 0) parent[0] = -1;
 }
 
-// bottom-up boxes: one thread per leaf climbs; the second child to arrive at a node computes it
+// The bottom-up climb of both box fits: a thread that has finished a node's box (a leaf's, or an inner node's) fences
+// it and arrives at the parent, one arrival flag per inner node.  The first arrival stops, because the sibling subtree
+// is not ready yet; the second one fits the parent from both children, first child then second, reading the sibling's
+// box past L1 (another SM may have written it), fences it and climbs on.
+template <class Fit>
+__device__ __forceinline__ void climb_boxes(int node, const int* __restrict__ parent, int* flags, Fit fit) {
+  while (node >= 0) {
+    if (atomicAdd(&flags[node], 1) == 0) return;  // first arrival: the sibling subtree is not ready yet
+    __threadfence();
+    fit(node);
+    __threadfence();
+    node = parent[node];
+  }
+}
+
+// LBVH boxes: one thread per leaf climbs; the second child to arrive at a node computes it
 __global__ void k_fit_boxes(const RefPrim* __restrict__ prims, const int* __restrict__ order, int n,
                             const int2* __restrict__ children, const int* __restrict__ parent, float* boxes,
                             int* flags) {
   int j = blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= n) return;
-  int node = parent[n - 1 + j];
-  while (node >= 0) {
-    if (atomicAdd(&flags[node], 1) == 0) return;  // first arrival: the sibling subtree is not ready yet
-    __threadfence();
+  climb_boxes(parent[n - 1 + j], parent, flags, [&](int node) {
     float mn[3] = {FLT_MAX, FLT_MAX, FLT_MAX}, mx[3] = {-FLT_MAX, -FLT_MAX, -FLT_MAX};
     int2 ch = children[node];
     int refs[2] = {ch.x, ch.y};
@@ -247,9 +259,69 @@ __global__ void k_fit_boxes(const RefPrim* __restrict__ prims, const int* __rest
       boxes[6 * node + k] = mn[k];
       boxes[6 * node + 3 + k] = mx[k];
     }
-    __threadfence();
-    node = parent[node];
+  });
+}
+
+// ---- refit of a tree in the reference layout (lt_scene_refit) ----
+
+// std::min / std::max: the first operand on ties, so that of -0 and +0 the earlier one is kept, as the host builder
+// (acceleration_structure_explicit.cpp) and Model's primitive bounds compute them.  fminf / fmaxf promise no sign.
+__device__ __forceinline__ float first_min(float a, float b) { return b < a ? b : a; }
+__device__ __forceinline__ float first_max(float a, float b) { return a < b ? b : a; }
+
+// parent of every node of a DFS-layout tree: inner node i has children i + 1 and offset
+__global__ void k_dfs_parents(const RefNode* __restrict__ nodes, int n, int* parent) {
+  int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  if (i == 0) parent[0] = -1;
+  if (nodes[i].primitiveCount == 0) {
+    parent[i + 1] = i;
+    parent[nodes[i].offset] = i;
   }
+}
+
+// One thread per leaf: the leaf's box covers all primitiveCount primitives from its offset, in order; then the climb
+// fits every inner node from its first child (i + 1) and its second (offset), in that order.
+__global__ void k_refit(RefNode* nodes, int n, const RefPrim* __restrict__ prims, const int* __restrict__ parent,
+                        int* flags) {
+  int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int count = nodes[i].primitiveCount, first = nodes[i].offset;
+  if (count == 0) return;
+  float mn[3], mx[3];
+  for (int j = 0; j < count; j++) {
+    const RefPrim& p = prims[first + j];
+    for (int k = 0; k < 3; k++) {
+      const float lo = first_min(first_min(p.a[k], p.b[k]), p.c[k]);
+      const float hi = first_max(first_max(p.a[k], p.b[k]), p.c[k]);
+      mn[k] = j ? first_min(mn[k], lo) : lo;
+      mx[k] = j ? first_max(mx[k], hi) : hi;
+    }
+  }
+  for (int k = 0; k < 3; k++) {
+    nodes[i].boundsMin[k] = mn[k];
+    nodes[i].boundsMax[k] = mx[k];
+  }
+  __threadfence();
+  climb_boxes(parent[i], parent, flags, [&](int node) {
+    const volatile RefNode* a = nodes + node + 1;
+    const volatile RefNode* b = nodes + nodes[node].offset;
+    for (int k = 0; k < 3; k++) {
+      nodes[node].boundsMin[k] = first_min(a->boundsMin[k], b->boundsMin[k]);
+      nodes[node].boundsMax[k] = first_max(a->boundsMax[k], b->boundsMax[k]);
+    }
+  });
+}
+
+// bad |= 1 for a materialIndex outside [0, matCount), |= 2 for a non-finite vertex coordinate
+__global__ void k_check_prims(const RefPrim* __restrict__ prims, int n, int matCount, int* bad) {
+  int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const RefPrim& p = prims[i];
+  int why = p.materialIndex < 0 || p.materialIndex >= matCount ? 1 : 0;
+  for (int k = 0; k < 3; k++)
+    if (!isfinite(p.a[k]) || !isfinite(p.b[k]) || !isfinite(p.c[k])) why |= 2;
+  if (why) atomicOr(bad, why);
 }
 
 // ---- PLOC iteration over the cluster array of length m ----
@@ -487,6 +559,24 @@ __global__ void k_flag_emissive(const RefPrim* __restrict__ orderedPrims, int n,
 }
 
 }  // namespace
+
+int lt_launch_refit_parents(const RefNode* dNodes, int n, int* dParent, cudaStream_t stream) {
+  k_dfs_parents<<<(n + 255) / 256, 256, 0, stream>>>(dNodes, n, dParent);
+  return 1;
+}
+
+int lt_launch_refit(RefNode* dNodes, int n, const RefPrim* dPrims, const int* dParent, int* dFlags,
+                    cudaStream_t stream) {
+  cudaMemsetAsync(dFlags, 0, sizeof(int) * (size_t)n, stream);
+  k_refit<<<(n + 255) / 256, 256, 0, stream>>>(dNodes, n, dPrims, dParent, dFlags);
+  return 1;
+}
+
+int lt_launch_check_prims(const RefPrim* dPrims, int n, int matCount, int* dBad, cudaStream_t stream) {
+  cudaMemsetAsync(dBad, 0, sizeof(int), stream);
+  k_check_prims<<<(n + 255) / 256, 256, 0, stream>>>(dPrims, n, matCount, dBad);
+  return 1;
+}
 
 size_t lt_bvh_scratch_bytes(int n, LtBvhBuilder builder) {
   BuildScratch S;

@@ -109,6 +109,20 @@ int lt_internal_fail(lt_ctx* ctx, int code, const std::string& msg) { return fai
 
 int lt_internal_ctx_device(const lt_ctx* ctx) { return ctx->device; }
 
+// cudaMalloc / cudaFree of a buffer the scene owns, counted in s->deviceBytes (lt_debug_scene_bytes)
+template <class T>
+static cudaError_t scene_alloc(lt_scene* s, T** p, size_t bytes) {
+  const cudaError_t e = cudaMalloc((void**)p, bytes);
+  if (e == cudaSuccess) s->deviceBytes += bytes;
+  return e;
+}
+template <class T>
+static void scene_free(lt_scene* s, T** p, size_t bytes) {
+  if (*p) s->deviceBytes -= bytes;
+  cudaFree(*p);
+  *p = nullptr;
+}
+
 // ------------------------------------------------------------------------------------------------
 // Launch plan: which kernels a call runs, on which tree, at which sizes.  Pure (no CUDA call, no allocation), so that
 // lt_debug_plan shows it on a machine without a GPU.
@@ -407,6 +421,7 @@ extern "C" void lt_scene_release(lt_ctx* ctx, lt_scene* s) {
   cudaFree(s->dThread);
   cudaFree(s->dRank);
   cudaFree(s->dThreadBig);
+  cudaFree(s->dRefit);
   delete s;
 }
 
@@ -1197,8 +1212,72 @@ extern "C" int lt_debug_scene_full_threaded(lt_scene* scene, int full) {
   return LT_OK;
 }
 
-// Re-flatten on the device (inner-node ranks -> 64-byte child-pair nodes, 48-byte triangles) and fill the
-// device-side scene descriptor.  ev0 must already be recorded on the stream; on failure the scene is released.
+// The buffers derived from dNodes and dPrims, written into the scene's allocations: the 64-byte child-pair nodes and
+// 48-byte triangles (re-flatten through the inner-node ranks dInnerRank), the threaded copies the scene keeps
+// (`copies`: built on the host for small trees, the one pass that may grow dThread or add dRank, or on the device for
+// large ones), and the launch state.  Upload and refit share it, so a refitted scene is what an upload of its buffers
+// makes.  ev0 must already be recorded on the stream; records ev1 and sets upload_ms.
+static cudaError_t derive_scene(lt_ctx* ctx, lt_scene* s, const int* dInnerRank, LtTree copies, const RefNode& root) {
+  LtSceneDev& d = s->dev;
+  const int nNodes = d.nodeCount, nPrims = d.primCount;
+  cudaError_t e = cudaSuccess;
+  auto A = [&](cudaError_t r) { if (e == cudaSuccess) e = r; };
+  cudaStream_t st = ctx->stream;
+  lt_launch_reflatten(s->dNodes, nNodes, s->dPrims, nPrims, dInnerRank, s->dWide, s->dTris, st);
+  A(cudaGetLastError());
+  std::vector<int> hRank;
+  if (e == cudaSuccess && copies == LT_TREE_HOST_THREADED) {
+    std::vector<RefNode> hNodes((size_t)nNodes);
+    std::vector<LtThreadNode> hThread;
+    A(cudaMemcpyAsync(hNodes.data(), s->dNodes, sizeof(RefNode) * (size_t)nNodes, cudaMemcpyDeviceToHost, st));
+    A(cudaStreamSynchronize(st));
+    if (e == cudaSuccess) {
+      s->threadStride = build_threaded(hNodes.data(), nNodes, nPrims, hThread, hRank);
+      if (hThread.size() > s->threadRecords) {  // the pruned copies' size follows the boxes
+        scene_free(s, &s->dThread, sizeof(LtThreadNode) * s->threadRecords);
+        s->threadRecords = 0;
+        A(scene_alloc(s, &s->dThread, sizeof(LtThreadNode) * hThread.size()));
+        if (e == cudaSuccess) s->threadRecords = hThread.size();
+      }
+      A(cudaMemcpyAsync(s->dThread, hThread.data(), sizeof(LtThreadNode) * hThread.size(), cudaMemcpyHostToDevice, st));
+      if (!hRank.empty()) {
+        if (!s->dRank) A(scene_alloc(s, &s->dRank, sizeof(int) * hRank.size()));
+        A(cudaMemcpyAsync(s->dRank, hRank.data(), sizeof(int) * hRank.size(), cudaMemcpyHostToDevice, st));
+      }
+      A(cudaStreamSynchronize(st));  // hThread and hRank are pageable and go out of scope
+    }
+  }
+  // large trees: the threaded copies are built on the device and used by coherent-ray launches only (plan_tree)
+  if (e == cudaSuccess && copies == LT_TREE_DEVICE_THREADED) {
+    if (!s->dThreadBig && scene_alloc(s, &s->dThreadBig, sizeof(LtThreadNode) * 8 * (size_t)nNodes) != cudaSuccess) {
+      cudaGetLastError();  // no memory for the copies: the stack traversal serves every launch
+      s->dThreadBig = nullptr;
+    }
+    if (s->dThreadBig) {
+      lt_launch_build_threaded(s->dNodes, nNodes, s->dThreadBig, st);
+      A(cudaGetLastError());
+    }
+  }
+  A(cudaEventRecord(ctx->ev1, st));
+  A(cudaStreamSynchronize(st));
+  if (e != cudaSuccess) return e;
+  cudaEventElapsedTime(&ctx->stats.upload_ms, ctx->ev0, ctx->ev1);
+  d.wnodes = s->dWide;
+  d.tris = s->dTris;
+  for (int k = 0; k < 3; k++) {
+    d.rootMin[k] = root.boundsMin[k];
+    d.rootMax[k] = root.boundsMax[k];
+  }
+  d.rootRef = root.primitiveCount > 0 ? ~root.offset : 0;  // inner root is wide node 0
+  d.rootCount = root.primitiveCount;
+  d.tnodes = s->dThread;
+  d.rank = hRank.empty() ? nullptr : s->dRank;
+  set_pruned_copies(s, false);
+  return cudaSuccess;
+}
+
+// Allocates the re-flattened buffers, derives them (derive_scene) and fills the device-side scene descriptor.  ev0
+// must already be recorded on the stream; on failure the scene is released.
 static int finish_scene(lt_ctx* ctx, lt_scene* s, int nNodes, int nPrims, int nMats, const RefNode& root,
                         int stackDepth, const char* who) {
   int* dFlags = nullptr;
@@ -1207,50 +1286,29 @@ static int finish_scene(lt_ctx* ctx, lt_scene* s, int nNodes, int nPrims, int nM
   int nInner = (nNodes - 1) / 2;  // a full binary tree with one primitive slot per leaf
   if (nNodes == 1) nInner = 0;
   size_t tempBytes = lt_scan_temp_bytes(nNodes);
+  LtSceneDev& d = s->dev;
+  d.prims = s->dPrims;
+  d.mats = s->dMats;
+  d.lights = s->dLights;
+  d.stackDepth = stackDepth;
+  d.nodeCount = nNodes;
+  d.primCount = nPrims;
+  d.matCount = nMats;
   cudaError_t e = cudaSuccess;
   auto A = [&](cudaError_t r) { if (e == cudaSuccess) e = r; };
   cudaStream_t st = ctx->stream;
-  A(cudaMalloc(&s->dWide, sizeof(LtWideNode) * (size_t)(nInner > 0 ? nInner : 1)));
-  A(cudaMalloc(&s->dTris, sizeof(LtTri) * (size_t)nPrims));
+  A(scene_alloc(s, &s->dWide, sizeof(LtWideNode) * (size_t)(nInner > 0 ? nInner : 1)));
+  A(scene_alloc(s, &s->dTris, sizeof(LtTri) * (size_t)nPrims));
   A(cudaMalloc(&dFlags, sizeof(int) * (size_t)nNodes));
   A(cudaMalloc(&dRank, sizeof(int) * (size_t)nNodes));
   A(cudaMalloc(&dTemp, tempBytes ? tempBytes : 16));
   if (e == cudaSuccess) {
     lt_launch_inner_flags(s->dNodes, nNodes, dFlags, st);
     lt_launch_exclusive_scan(dTemp, tempBytes, dFlags, dRank, nNodes, st);
-    lt_launch_reflatten(s->dNodes, nNodes, s->dPrims, nPrims, dRank, s->dWide, s->dTris, st);
     A(cudaGetLastError());
   }
-  const LtTree copies = lt_plan_threaded_copies(nNodes, ctx->totalMem, ctx->limits);
-  if (e == cudaSuccess && copies == LT_TREE_HOST_THREADED) {
-    std::vector<RefNode> hNodes((size_t)nNodes);
-    std::vector<LtThreadNode> hThread;
-    std::vector<int> hRank;
-    A(cudaMemcpyAsync(hNodes.data(), s->dNodes, sizeof(RefNode) * (size_t)nNodes, cudaMemcpyDeviceToHost, st));
-    A(cudaStreamSynchronize(st));
-    if (e == cudaSuccess) {
-      s->threadStride = build_threaded(hNodes.data(), nNodes, nPrims, hThread, hRank);
-      A(cudaMalloc(&s->dThread, sizeof(LtThreadNode) * hThread.size()));
-      A(cudaMemcpyAsync(s->dThread, hThread.data(), sizeof(LtThreadNode) * hThread.size(), cudaMemcpyHostToDevice, st));
-      if (!hRank.empty()) {
-        A(cudaMalloc(&s->dRank, sizeof(int) * hRank.size()));
-        A(cudaMemcpyAsync(s->dRank, hRank.data(), sizeof(int) * hRank.size(), cudaMemcpyHostToDevice, st));
-      }
-      A(cudaStreamSynchronize(st));  // hThread and hRank are pageable and go out of scope
-    }
-  }
-  // large trees: the threaded copies are built on the device and used by coherent-ray launches only (plan_tree)
-  if (e == cudaSuccess && copies == LT_TREE_DEVICE_THREADED) {
-    if (cudaMalloc(&s->dThreadBig, sizeof(LtThreadNode) * 8 * (size_t)nNodes) == cudaSuccess) {
-      lt_launch_build_threaded(s->dNodes, nNodes, s->dThreadBig, st);
-      A(cudaGetLastError());
-    } else {
-      cudaGetLastError();  // no memory for the copies: the stack traversal serves every launch
-      s->dThreadBig = nullptr;
-    }
-  }
-  A(cudaEventRecord(ctx->ev1, st));
-  A(cudaStreamSynchronize(st));
+  if (e == cudaSuccess) A(derive_scene(ctx, s, dRank, lt_plan_threaded_copies(nNodes, ctx->totalMem, ctx->limits), root));
+  cudaStreamSynchronize(st);
   cudaFree(dFlags);
   cudaFree(dRank);
   cudaFree(dTemp);
@@ -1258,26 +1316,6 @@ static int finish_scene(lt_ctx* ctx, lt_scene* s, int nNodes, int nPrims, int nM
     lt_scene_release(ctx, s);
     return fail(ctx, LT_ERR_CUDA, std::string(who) + ": " + cudaGetErrorString(e));
   }
-  cudaEventElapsedTime(&ctx->stats.upload_ms, ctx->ev0, ctx->ev1);
-  LtSceneDev& d = s->dev;
-  d.wnodes = s->dWide;
-  d.tris = s->dTris;
-  d.prims = s->dPrims;
-  d.mats = s->dMats;
-  d.lights = s->dLights;
-  for (int k = 0; k < 3; k++) {
-    d.rootMin[k] = root.boundsMin[k];
-    d.rootMax[k] = root.boundsMax[k];
-  }
-  d.rootRef = root.primitiveCount > 0 ? ~root.offset : 0;  // inner root is wide node 0
-  d.rootCount = root.primitiveCount;
-  d.stackDepth = stackDepth;
-  d.nodeCount = nNodes;
-  d.primCount = nPrims;
-  d.matCount = nMats;
-  d.tnodes = s->dThread;
-  d.rank = s->dRank;
-  set_pruned_copies(s, false);
   return LT_OK;
 }
 
@@ -1315,10 +1353,10 @@ static int build_scene_on_device(lt_ctx* ctx, LtBvhBuilder builder, const char* 
   size_t scratchBytes = lt_bvh_scratch_bytes(n, builder);
   cudaError_t e = cudaSuccess;
   auto A = [&](cudaError_t r) { if (e == cudaSuccess) e = r; };
-  A(cudaMalloc(&s->dNodes, sizeof(RefNode) * (size_t)nNodes));
-  A(cudaMalloc(&s->dPrims, primitive_bytes));
-  A(cudaMalloc(&s->dMats, material_bytes));
-  A(cudaMalloc(&s->dLights, sizeof(RefLights)));
+  A(scene_alloc(s, &s->dNodes, sizeof(RefNode) * (size_t)nNodes));
+  A(scene_alloc(s, &s->dPrims, primitive_bytes));
+  A(scene_alloc(s, &s->dMats, material_bytes));
+  A(scene_alloc(s, &s->dLights, sizeof(RefLights)));
   A(cudaMalloc(&dInput, primitive_bytes));
   A(cudaMalloc(&scratch, scratchBytes));
   cudaStream_t st = ctx->stream;
@@ -1427,10 +1465,10 @@ extern "C" int lt_scene_upload(lt_ctx* ctx, const void* nodes, uint64_t node_byt
   lt_scene* s = new lt_scene();
   cudaError_t e = cudaSuccess;
   auto A = [&](cudaError_t r) { if (e == cudaSuccess) e = r; };
-  A(cudaMalloc(&s->dNodes, node_bytes));
-  A(cudaMalloc(&s->dPrims, primitive_bytes));
-  A(cudaMalloc(&s->dMats, material_bytes ? material_bytes : sizeof(RefMaterial)));
-  A(cudaMalloc(&s->dLights, sizeof(RefLights)));
+  A(scene_alloc(s, &s->dNodes, node_bytes));
+  A(scene_alloc(s, &s->dPrims, primitive_bytes));
+  A(scene_alloc(s, &s->dMats, material_bytes ? material_bytes : sizeof(RefMaterial)));
+  A(scene_alloc(s, &s->dLights, sizeof(RefLights)));
   cudaStream_t st = ctx->stream;
   A(cudaEventRecord(ctx->ev0, st));
   A(cudaMemcpyAsync(s->dNodes, nodes, node_bytes, cudaMemcpyHostToDevice, st));
@@ -1502,6 +1540,125 @@ static LtSceneDev scene_for_plan(const lt_scene* s, const LtPlan& plan) {
   return d;
 }
 
+// Both forms of lt_scene_refit, after the checks that need no device: `src` holds the scene's primitive count of new
+// primitives in host memory, already checked, or in device memory (onDevice), checked here by a kernel.  Nothing of
+// the scene is written before every check has passed.  The topology's parents and inner-node ranks are derived on the
+// first refit that passes them, and kept.
+static int refit_scene(lt_ctx* ctx, lt_scene* s, const void* src, bool onDevice, const char* who) {
+  const std::string w = std::string(who) + ": ";
+  CK(cudaSetDevice(ctx->device));
+  const int n = s->dev.nodeCount, nPrims = s->dev.primCount;
+  cudaStream_t st = ctx->stream;
+  if (onDevice) {
+    cudaPointerAttributes pa;
+    if (cudaPointerGetAttributes(&pa, src) != cudaSuccess ||
+        (pa.type != cudaMemoryTypeDevice && pa.type != cudaMemoryTypeManaged) || pa.device != ctx->device) {
+      cudaGetLastError();
+      return fail(ctx, LT_ERR_INVALID, w + "device_primitives is not device memory of the context's device");
+    }
+    if ((uintptr_t)src % alignof(RefPrim))
+      return fail(ctx, LT_ERR_INVALID, w + "device_primitives is not 4-byte aligned");
+  }
+  // The upload checks only a leaf's first primitive (the reference's leaves test no other, SURVEY H1); the refit reads
+  // all of them, so every leaf's range must lie in the primitive buffer.
+  if (s->refitLeaves == 0) {
+    std::vector<RefNode> hNodes((size_t)n);
+    CK(cudaMemcpyAsync(hNodes.data(), s->dNodes, sizeof(RefNode) * (size_t)n, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    s->refitLeaves = 1;
+    for (const RefNode& r : hNodes)
+      if (r.primitiveCount > 0 && (long long)r.offset + r.primitiveCount > nPrims) s->refitLeaves = -1;
+  }
+  if (s->refitLeaves < 0)
+    return fail(ctx, LT_ERR_INVALID, w + "a leaf's primitives run past the primitive buffer: the scene cannot be refitted");
+  if (!s->dRefit) CK(scene_alloc(s, &s->dRefit, sizeof(int) * (3 * (size_t)n + 1)));
+  int *parent = s->dRefit, *flags = parent + n, *rank = flags + n, *bad = rank + n;
+  if (onDevice) {
+    lt_launch_check_prims((const RefPrim*)src, nPrims, s->dev.matCount, bad, st);
+    int why = 0;
+    CK(cudaMemcpyAsync(&why, bad, sizeof why, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (why & 1) return fail(ctx, LT_ERR_INVALID, w + "primitive materialIndex out of range");
+    if (why) return fail(ctx, LT_ERR_INVALID, w + "non-finite vertex coordinate");
+  }
+  if (!s->refitDerived) {  // the inner-node ranks as the upload computes them, with the arrival flags as the scan's input
+    // Host-built copies: room for the largest pruned copies (8 n records besides the full ones) and for the tie-break
+    // table, so that no later refit allocates whatever the boxes do to the traversal tree.
+    if (s->dThread && s->threadRecords < 16 * (size_t)n) {
+      CK(cudaStreamSynchronize(st));
+      scene_free(s, &s->dThread, sizeof(LtThreadNode) * s->threadRecords);
+      s->threadRecords = 0;
+      s->dev.tnodes = nullptr;
+      CK(scene_alloc(s, &s->dThread, sizeof(LtThreadNode) * 16 * (size_t)n));
+      s->threadRecords = 16 * (size_t)n;
+    }
+    if (s->dThread && !s->dRank) CK(scene_alloc(s, &s->dRank, sizeof(int) * 8 * (size_t)nPrims));
+    void* dTemp = nullptr;
+    const size_t tempBytes = lt_scan_temp_bytes(n);
+    CK(cudaMalloc(&dTemp, tempBytes ? tempBytes : 16));
+    lt_launch_refit_parents(s->dNodes, n, parent, st);
+    lt_launch_inner_flags(s->dNodes, n, flags, st);
+    lt_launch_exclusive_scan(dTemp, tempBytes, flags, rank, n, st);
+    const cudaError_t e = cudaStreamSynchronize(st);
+    cudaFree(dTemp);
+    CK(e);
+    s->refitDerived = true;
+  }
+  CK(cudaEventRecord(ctx->ev0, st));
+  CK(cudaMemcpyAsync(s->dPrims, src, sizeof(RefPrim) * (size_t)nPrims,
+                     onDevice ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, st));
+  lt_launch_refit(s->dNodes, n, s->dPrims, parent, flags, st);
+  CK(cudaGetLastError());
+  RefNode root;
+  CK(cudaMemcpyAsync(&root, s->dNodes, sizeof root, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));  // the root box travels in the launch state
+  const cudaError_t e = derive_scene(ctx, s, rank, scene_facts(s).copies, root);
+  if (e != cudaSuccess) return fail(ctx, LT_ERR_CUDA, w + cudaGetErrorString(e));
+  return LT_OK;
+}
+int lt_internal_refit(lt_ctx* ctx, lt_scene* scene, const void* primitives) {
+  return refit_scene(ctx, scene, primitives, false, "lt_scene_refit");
+}
+
+// the checks of both forms that need no device; prims: host primitives to check, or NULL
+static int refit_args(lt_ctx* ctx, const lt_scene* scene, const void* prims, uint64_t primitive_bytes,
+                      const RefPrim* hostPrims, const char* who) {
+  const std::string w = std::string(who) + ": ";
+  if (!ctx) return fail(nullptr, LT_ERR_INVALID, w + "ctx is NULL");
+  if (!scene || !prims) return fail(ctx, LT_ERR_INVALID, w + "NULL argument");
+  if (!scene->parts.empty() != (ctx->group != nullptr))
+    return fail(ctx, LT_ERR_INVALID, w + "the scene was not uploaded to this context");
+  const lt_scene* one = scene->parts.empty() ? scene : scene->parts[0];
+  const uint64_t nPrims = (uint64_t)one->dev.primCount;
+  if (primitive_bytes != sizeof(RefPrim) * nPrims)
+    return fail(ctx, LT_ERR_INVALID, w + "primitive_bytes is not the scene's primitive count x 76");
+  if (hostPrims) {
+    for (uint64_t i = 0; i < nPrims; i++)
+      if (hostPrims[i].materialIndex < 0 || hostPrims[i].materialIndex >= one->dev.matCount)
+        return fail(ctx, LT_ERR_INVALID, w + "primitive materialIndex out of range");
+    for (uint64_t i = 0; i < nPrims; i++)
+      for (int k = 0; k < 3; k++)
+        if (!std::isfinite(hostPrims[i].a[k]) || !std::isfinite(hostPrims[i].b[k]) || !std::isfinite(hostPrims[i].c[k]))
+          return fail(ctx, LT_ERR_INVALID, w + "non-finite vertex coordinate");
+  }
+  return LT_OK;
+}
+
+extern "C" int lt_scene_refit(lt_ctx* ctx, lt_scene* scene, const void* primitives, uint64_t primitive_bytes) {
+  const char* who = "lt_scene_refit";
+  if (int rc = refit_args(ctx, scene, primitives, primitive_bytes, (const RefPrim*)primitives, who)) return rc;
+  if (ctx->group) return lt_multi_scene_refit(ctx, scene, primitives);
+  return refit_scene(ctx, scene, primitives, false, who);
+}
+
+extern "C" int lt_scene_refit_device(lt_ctx* ctx, lt_scene* scene, const void* device_primitives,
+                                     uint64_t primitive_bytes) {
+  const char* who = "lt_scene_refit_device";
+  if (ctx && ctx->group) return fail(ctx, LT_ERR_UNSUPPORTED, std::string(who) + ": single-GPU contexts only");
+  if (int rc = refit_args(ctx, scene, device_primitives, primitive_bytes, nullptr, who)) return rc;
+  return refit_scene(ctx, scene, device_primitives, true, who);
+}
+
 static int debug_plan(const char* who, const lt_render_params* params, int views, uint64_t node_count,
                       int32_t stack_depth, uint64_t total_mem, int32_t sm_count, int64_t* out) {
   if (!params || !out || views < 1 || node_count < 1 || node_count > 0x7fffffffull || sm_count < 1)
@@ -1526,6 +1683,14 @@ extern "C" int lt_debug_plan(const lt_render_params* params, uint64_t node_count
 extern "C" int lt_debug_plan_views(const lt_render_params* params, int view_count, uint64_t node_count,
                                    int32_t stack_depth, uint64_t total_mem, int32_t sm_count, int64_t* out) {
   return debug_plan("lt_debug_plan_views", params, view_count, node_count, stack_depth, total_mem, sm_count, out);
+}
+
+extern "C" int lt_debug_scene_bytes(const lt_scene* scene, uint64_t* out_bytes) {
+  if (!scene || !out_bytes) return fail(nullptr, LT_ERR_INVALID, "lt_debug_scene_bytes: NULL argument");
+  uint64_t bytes = 0;
+  for (const lt_scene* p : scene->parts) bytes += p->deviceBytes;
+  *out_bytes = scene->parts.empty() ? scene->deviceBytes : bytes;
+  return LT_OK;
 }
 
 extern "C" int lt_debug_ctx_limits(lt_ctx* ctx, int threaded_max_nodes, int stream_min_nodes) {

@@ -183,9 +183,14 @@ struct lt_scene {
   LtWideNode* dWide = nullptr;
   LtTri* dTris = nullptr;
   LtThreadNode* dThread = nullptr;  // 8 octant copies in visit order, then 8 pruned ones, small scenes only
+  size_t threadRecords = 0;         // records allocated at dThread
   int threadStride = 0;             // records per pruned copy
   int* dRank = nullptr;             // LtSceneDev::rank, when the pruned copies are a traversal tree
   LtThreadNode* dThreadBig = nullptr;  // the same for a large scene, built on the device, for coherent-ray launches
+  int* dRefit = nullptr;  // from the first lt_scene_refit on: parents, arrival flags, inner-node ranks (n each), check flag
+  bool refitDerived = false;  // dRefit holds the parents and the inner-node ranks
+  int refitLeaves = 0;        // 1: every leaf's primitive range lies in the primitive buffer, -1: not, 0: not checked
+  size_t deviceBytes = 0;     // device memory the scene holds (lt_debug_scene_bytes)
   LtSceneDev dev = {};
 };
 
@@ -195,6 +200,9 @@ int lt_multi_scene_upload(lt_ctx* ctx, const void* nodes, uint64_t node_bytes, c
                           uint64_t primitive_bytes, const void* materials, uint64_t material_bytes,
                           const void* light_container, uint64_t light_bytes, lt_scene** out_scene);
 void lt_multi_scene_release(lt_ctx* ctx, lt_scene* scene);
+// lt_scene_refit on every device's copy (arguments already checked)
+int lt_internal_refit(lt_ctx* ctx, lt_scene* scene, const void* primitives);  // one copy, host primitives checked
+int lt_multi_scene_refit(lt_ctx* ctx, lt_scene* scene, const void* primitives);
 // run: NULL renders the built-in kernel of params, otherwise the plug-in of run (loaded on every device)
 int lt_multi_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params, float* host_out,
                     const LtPluginRun* run);
@@ -226,3 +234,10 @@ size_t lt_bvh_scratch_bytes(int n, LtBvhBuilder builder);
 int lt_launch_bvh_build(LtBvhBuilder builder, const RefPrim* dPrims, int n, const RefMaterial* dMats, int matCount,
                         RefNode* dNodes, RefPrim* dOrderedPrims, RefLights* dLights, void* scratch, size_t scratchBytes,
                         int* outMaxDepth, cudaStream_t stream);
+// refit of a tree in the reference layout (lt_scene_refit): dParent receives every node's parent (-1 for the root);
+// the refit then fits every node's box to dPrims bottom-up, with one arrival flag per node in dFlags
+int lt_launch_refit_parents(const RefNode* dNodes, int n, int* dParent, cudaStream_t stream);
+int lt_launch_refit(RefNode* dNodes, int n, const RefPrim* dPrims, const int* dParent, int* dFlags,
+                    cudaStream_t stream);
+// *dBad = 0, then |= 1 for a materialIndex outside [0, matCount) and |= 2 for a non-finite vertex coordinate
+int lt_launch_check_prims(const RefPrim* dPrims, int n, int matCount, int* dBad, cudaStream_t stream);

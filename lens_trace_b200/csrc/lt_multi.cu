@@ -200,6 +200,22 @@ int lt_multi_scene_upload(lt_ctx* ctx, const void* nodes, uint64_t node_bytes, c
   return LT_OK;
 }
 
+int lt_multi_scene_refit(lt_ctx* ctx, lt_scene* scene, const void* primitives) {
+  LtGroup* g = ctx->group;
+  std::vector<int> rcs(g->ctx.size(), LT_OK);
+  std::vector<std::thread> workers;
+  for (size_t k = 0; k < g->ctx.size(); k++)
+    workers.emplace_back([&, k]() { rcs[k] = lt_internal_refit(g->ctx[k], scene->parts[k], primitives); });
+  for (std::thread& t : workers) t.join();
+  float ms = 0.0f;
+  for (size_t k = 0; k < g->ctx.size(); k++)
+    if (g->ctx[k]->stats.upload_ms > ms) ms = g->ctx[k]->stats.upload_ms;
+  ctx->stats.upload_ms = ms;
+  for (size_t k = 0; k < g->ctx.size(); k++)
+    if (rcs[k] != LT_OK) return lt_internal_fail(ctx, rcs[k], lt_last_error(g->ctx[k]));
+  return LT_OK;
+}
+
 void lt_multi_scene_release(lt_ctx* ctx, lt_scene* scene) {
   LtGroup* g = ctx ? ctx->group : nullptr;
   for (size_t k = 0; k < scene->parts.size(); k++)
