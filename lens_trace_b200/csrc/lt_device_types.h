@@ -4,7 +4,7 @@
 #include "lens_trace_b200_device.cuh"  // buffer layouts
 
 // The values of enum lt_kernel and enum lt_flags (include/lens_trace_b200.h) that the device code tests: NVRTC cannot
-// include the public header.  lt_capi.cu checks that both agree.
+// include the public header.  lt_plan.cpp checks that both agree.
 constexpr int LT_DEV_KERNEL_BASIC_CU = 0;
 constexpr int LT_DEV_KERNEL_BASIC_CL = 1;
 constexpr int LT_DEV_KERNEL_CUSTOM_BARY = 2;

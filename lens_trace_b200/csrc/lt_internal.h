@@ -4,6 +4,11 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <string>
+#include <utility>
+#include <vector>
+
+#include "lens_trace_b200.h"
 #include "lens_trace_b200_device.cuh"  // buffer layouts shared with plug-in kernels
 
 #include "lt_device_types.h"  // LtLaunch, LtCounters (shared with plug-in builds)
@@ -11,7 +16,7 @@
 struct lt_ctx;
 int lt_internal_ctx_device(const lt_ctx* ctx);  // lt_capi.cu
 
-// ---- launch plan (lt_capi.cu: lt_plan_render): every choice of which kernels run, on which tree, at which sizes ----
+// ---- launch plan (lt_plan.cpp: lt_plan_render): every choice of which kernels run, on which tree, at which sizes ----
 // k_flat, k_flat_stream, k_path, or the wavefront pipeline (lt_wavefront.cu)
 enum LtPipeline { LT_PIPE_FLAT, LT_PIPE_FLAT_STREAM, LT_PIPE_PATH, LT_PIPE_WAVEFRONT };
 // the tree the traversal kernels walk: child-pair nodes with a stack, or the host- or device-built threaded copies
@@ -38,6 +43,28 @@ struct LtPlan {
   int blocksPerSm;      // persistent kernels (k_flat_stream, k_wf_trace)
   int grid;             // blocks: persistent grid, or one block per 16x8 tile (k_flat, k_path)
 };
+struct LtSceneFacts {
+  int nodeCount, stackDepth;
+  LtTree copies;  // the threaded copies the scene has (LT_TREE_CHILD_PAIR: none)
+};
+LtTree lt_plan_threaded_copies(int nNodes, size_t totalMem, const LtLimits& lim);
+LtPlan lt_plan_primary_hits(int flags, int width, int height, const LtSceneFacts& s);
+LtPlan lt_plan_render(const LtLaunch& L, const LtSceneFacts& s, size_t totalMem, int smCount, const LtLimits& lim,
+                      int views = 1);
+// The struct-size check of a caller's lt_render_params and its zero-filled copy at *P, which has the current
+// struct_size; `w` starts the error message ("lt_render: ")
+int lt_params_normalise(lt_ctx* ctx, const lt_render_params* params, const std::string& w, lt_render_params* P);
+// lt_render_params -> the launch descriptor (all of it but the camera), with lt_render's checks; `who` names the entry
+// point in error messages
+int lt_params_to_launch(lt_ctx* ctx, const lt_render_params* params, LtLaunch* L, const char* who = "lt_render");
+
+// ---- host tree builders (lt_tree.cpp) ----
+// Host-side validation of the reference node array (bounds of every index the kernels will follow) and the depth the
+// traversal stack needs; nonzero with *why set when it fails.
+int lt_validate_tree(const RefNode* nodes, int nodeCount, int primCount, int* stackDepth, std::string* why);
+// The threaded copies lt_scene_upload makes of a small tree, and the rank table; returns the pruned stride.
+int lt_build_threaded(const RefNode* nodes, int n, int primCount, std::vector<LtThreadNode>& out,
+                      std::vector<int>& rank);
 
 // launchers implemented in lt_kernels.cu (all asynchronous on `stream`; return launches made).  The launchers of the
 // traversal kernels take the scene with the plan's tree in `tnodes`.
@@ -92,9 +119,6 @@ int lt_launch_render_wavefront(const LtSceneDev& sc, const LtPlan& plan, const L
                                unsigned char* pairKinds, const LtWfAux* aux, const LtViews* views);
 
 // user-written CUDA kernels with the reference's plug-in ABI (lt_plugin.cu)
-#include <string>
-#include <utility>
-#include <vector>
 struct LtPlugin;
 // A compiled plug-in, not yet loaded on a device: compiled once, loaded on every device of a multi-GPU context.
 struct LtPluginImage {
@@ -135,8 +159,6 @@ struct LtPluginRun {
 };
 
 // ---- context and scene objects behind the C-ABI handles (lt_capi.cu; lt_multi.cu for multi-GPU contexts) ----
-#include <vector>
-#include "lens_trace_b200.h"
 struct LtGroup;     // lt_multi.cu: the devices of a multi-GPU context
 struct LtCopyPool;  // lt_capi.cu: host threads that copy staged chunks into a pageable destination
 

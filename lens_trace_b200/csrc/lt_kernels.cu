@@ -314,7 +314,7 @@ __global__ void k_build_wide(const RefNode* __restrict__ nodes, int n, const int
 }
 
 // Threaded form of a LARGE tree (LtThreadNode, see lens_trace_b200_device.cuh; small trees are threaded on the host,
-// lt_capi.cu: build_threaded): one thread per reference node walks from the root to its node through the
+// lt_tree.cpp: lt_build_threaded): one thread per reference node walks from the root to its node through the
 // depth-first index ranges (the left subtree of inner node i is [i+1, offset), the right one [offset, end)) and
 // accumulates, for all eight sign octants at once, the node's position in that octant's visit order -- descending
 // into the child the octant visits second skips the whole subtree of the one it visits first.

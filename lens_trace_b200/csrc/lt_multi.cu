@@ -360,12 +360,8 @@ int lt_multi_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt
   if (!scene || !camera28 || !params) return lt_internal_fail(ctx, LT_ERR_INVALID, who + "NULL argument");
   if (scene->parts.size() != g->ctx.size())
     return lt_internal_fail(ctx, LT_ERR_INVALID, who + "the scene was not uploaded through this multi-GPU context");
-  if (params->struct_size != sizeof(lt_render_params) && params->struct_size != offsetof(lt_render_params, split_mode))
-    return lt_internal_fail(ctx, LT_ERR_INVALID, who + "params.struct_size mismatch");
   lt_render_params P;
-  memset(&P, 0, sizeof P);
-  memcpy(&P, params, params->struct_size < sizeof P ? params->struct_size : sizeof P);
-  P.struct_size = sizeof P;
+  if (int rc = lt_params_normalise(ctx, params, who, &P)) return rc;
   if (P.width <= 0 || P.height <= 0 || P.depth < 3 || P.frames < 1)
     return lt_internal_fail(ctx, LT_ERR_INVALID, who + "width/height must be > 0, depth >= 3, frames >= 1");
   if (P.flags & LT_FLAG_STATS)
@@ -547,12 +543,8 @@ int lt_multi_render_views(lt_ctx* ctx, lt_scene* scene, const RefCamera* cams, i
   if (!scene || !params) return lt_internal_fail(ctx, LT_ERR_INVALID, who + "NULL argument");
   if (scene->parts.size() != g->ctx.size())
     return lt_internal_fail(ctx, LT_ERR_INVALID, who + "the scene was not uploaded through this multi-GPU context");
-  if (params->struct_size != sizeof(lt_render_params) && params->struct_size != offsetof(lt_render_params, split_mode))
-    return lt_internal_fail(ctx, LT_ERR_INVALID, who + "params.struct_size mismatch");
   lt_render_params P;
-  memset(&P, 0, sizeof P);
-  memcpy(&P, params, params->struct_size < sizeof P ? params->struct_size : sizeof P);
-  P.struct_size = sizeof P;
+  if (int rc = lt_params_normalise(ctx, params, who, &P)) return rc;
   if (P.split_mode != LT_SPLIT_AUTO)
     return lt_internal_fail(ctx, LT_ERR_INVALID, who + "views are dealt to the devices whole: split_mode must be LT_SPLIT_AUTO");
   if (P.flags & LT_FLAG_STATS)

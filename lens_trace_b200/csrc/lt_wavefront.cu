@@ -60,7 +60,7 @@ enum WfRound { WF_GENERIC, WF_FIRST_SHADOW, WF_SHADOW, WF_EXTENSION };
 __device__ __forceinline__ float* wf_dlight(const LtWfBuffers& B, int q) { return reinterpret_cast<float*>(B.payA[q]); }
 __device__ __forceinline__ int* wf_hit_words(const LtWfBuffers& B) { return reinterpret_cast<int*>(B.hits); }
 
-#define WF_PATH_BITS 25  // a batch holds at most 2^25 paths (lt_capi.cu caps it)
+#define WF_PATH_BITS 25  // a batch holds at most 2^25 paths (lt_plan.cpp caps it)
 __device__ __forceinline__ int wf_pack_path(int path, int stage, int depth) {
   return path | (stage << WF_PATH_BITS) | (depth << (WF_PATH_BITS + 2));
 }
