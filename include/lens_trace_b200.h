@@ -224,6 +224,36 @@ int lt_render_views(lt_ctx* ctx, lt_scene* scene, const void* cameras28, int vie
 int lt_render_views_device(lt_ctx* ctx, lt_scene* scene, const void* cameras28, int view_count,
                            const lt_render_params* params, float* device_out, int sync);
 
+/* lt_render_device for the pixels of a mask only: spend samples where the image is still noisy.
+ * device_mask: width * height bytes on ctx's device, row-major; a nonzero byte renders its pixel.  NULL: every pixel.
+ * Every masked pixel gets exactly what lt_render_device gives it: frames camera.frameCount + k * frame_stride for
+ * k < frames, combined by accum_mode into device_out from its current contents, bit for bit.  Pixels outside the mask
+ * are not written: their bytes in device_out and device_m2 stay as they were.  Every kernel id, accum_mode and flag of
+ * lt_render is accepted and means the same; with LT_FLAG_STATS the counters count the masked pixels' rays.
+ * A pixel's frame count is the caller's bookkeeping: camera.frameCount must be the number of frames the running mean
+ * of every masked pixel already holds.
+ * device_m2 (may be NULL): 3 floats per pixel (width * height * 3, whatever depth is) on ctx's device, the per-channel
+ * sum of squared deviations of the frame samples the running mean averages (Welford).  For a frame with frameCount n
+ * and sample x, in FP32 with one rounding per operation: n == 0 sets m2 = 0; n > 0 computes d = x - mean_prev, the
+ * running mean as always, then m2 = m2 + d * (x - mean).  The sample variance of a pixel of n frames is m2 / (n - 1).
+ * Only with LT_ACCUM_RUNNING_MEAN and frame_stride <= 1 (LT_ERR_INVALID otherwise).
+ * Checked before anything is launched: the parameters as lt_render; device_mask and device_m2 must be memory of ctx's
+ * device (LT_ERR_INVALID otherwise, device_m2 4-byte aligned); a multi-GPU context returns LT_ERR_UNSUPPORTED, and so
+ * does an image of more than 2^31 - 1 pixels (width * height): the pixel list holds 32-bit pixel indices.
+ * A kernel compacts the mask into a list of pixels in the context's memory (grow-only, like the wavefront workspace),
+ * and the launch plan is made for the listed pixels (lt_debug_plan_masked).  So with a mask the call reads the list's
+ * length back -- one 4-byte copy and a synchronisation of the context stream, the call's only one; otherwise it is
+ * asynchronous on the context stream unless sync != 0.  An empty mask launches nothing more and returns LT_OK.
+ * lt_last_stats describes the call as for lt_render_device; kernel_launches counts the compaction.
+ * Not provided: a host-memory form or the context accumulator, multi-GPU contexts, views, plug-ins, the C++ renderer
+ * (RenderExtensionB200), and any policy that chooses the mask: the caller decides which pixels need more frames. */
+int lt_render_masked_device(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params,
+                            const uint8_t* device_mask, float* device_out, float* device_m2, int sync);
+/* Test hook (single-GPU contexts): reversed != 0 makes later lt_render_masked_device calls on ctx render their pixel
+ * list in reverse order (one more kernel), 0 restores the compaction's order.  The output is the same either way; tests
+ * compare the two. */
+int lt_debug_ctx_list_order(lt_ctx* ctx, int reversed);
+
 /* The output buffer of the reference API is the caller's malloc'ed memory (pOutputBuffer, structures.h:62,76).
  * lt_render copies into such pageable memory through its own pinned staging buffer; an application that reuses one
  * buffer for many calls can page-lock it once instead, and the frame then arrives by a single DMA.  Unregister
@@ -334,6 +364,16 @@ int lt_debug_plan(const lt_render_params* params, uint64_t node_count, int32_t s
  * the primary records of every view one batch touches. */
 int lt_debug_plan_views(const lt_render_params* params, int view_count, uint64_t node_count, int32_t stack_depth,
                         uint64_t total_mem, int32_t sm_count, int64_t* out);
+/* Host-only: the plan of an lt_render_masked_device call whose mask lists pixel_count pixels (1 .. width * height), as
+ * lt_debug_plan.  Every size counts the listed pixels where lt_render counts the image's: the wavefront's threshold,
+ * frames per batch, its limit of 2^25 paths per frame, workspace and primary records, and the grids.  The
+ * deterministic kernels run k_flat over the list (pipeline 0, never k_flat_stream).  A partial list of the GI kernel
+ * (LT_KERNEL_GI, pixel_count < width * height) takes the wavefront from 2^20 paths, and from 2^16 paths at 16 frames
+ * or more: the crossovers measured for scattered pixels (DESIGN.md section 4).  Otherwise pixel_count = width *
+ * height plans exactly as lt_debug_plan.  An image of more than 2^31 - 1 pixels returns LT_ERR_UNSUPPORTED, as
+ * lt_render_masked_device does. */
+int lt_debug_plan_masked(const lt_render_params* params, int64_t pixel_count, uint64_t node_count, int32_t stack_depth,
+                         uint64_t total_mem, int32_t sm_count, int64_t* out);
 
 /* --- plug-in kernels: a user-written .cu file with the reference's kernel ABI (extern "C" __global__
  * linearKernel / tileKernel(LinearBVHNode*, Primitive*, Material*, LightContainer*, Camera*, float* out,

@@ -22,6 +22,7 @@ SYMBOLS = [
     "lt_debug_plan", "lt_debug_ctx_limits", "lt_render_plugin_frames", "lt_debug_build_traversal_tree",
     "lt_debug_scene_traversal_tree", "lt_debug_traversal_tree", "lt_render_views", "lt_render_views_device",
     "lt_debug_plan_views", "lt_scene_refit", "lt_scene_refit_device", "lt_debug_scene_bytes",
+    "lt_render_masked_device", "lt_debug_plan_masked", "lt_debug_ctx_list_order",
 ]
 
 
@@ -85,6 +86,9 @@ def load():
     lib.lt_render_views.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(RenderParams), C.c_void_p]
     lib.lt_render_views_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(RenderParams),
                                            C.c_void_p, C.c_int]
+    lib.lt_render_masked_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(RenderParams), C.c_void_p,
+                                            C.c_void_p, C.c_void_p, C.c_int]
+    lib.lt_debug_ctx_list_order.argtypes = [C.c_void_p, C.c_int]
     lib.lt_accum_reset.argtypes = [C.c_void_p]
     lib.lt_accum_read.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64]
     lib.lt_primary_hits.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p,
@@ -107,6 +111,8 @@ def load():
                                   C.POINTER(C.c_int64)]
     lib.lt_debug_plan_views.argtypes = [C.POINTER(RenderParams), C.c_int, C.c_uint64, C.c_int32, C.c_uint64, C.c_int32,
                                         C.POINTER(C.c_int64)]
+    lib.lt_debug_plan_masked.argtypes = [C.POINTER(RenderParams), C.c_int64, C.c_uint64, C.c_int32, C.c_uint64,
+                                         C.c_int32, C.POINTER(C.c_int64)]
     lib.lt_plugin_load.argtypes = [C.c_void_p, C.c_char_p, C.POINTER(C.c_int)]
     lib.lt_render_plugin.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                      C.c_int, C.c_int, C.c_void_p]
@@ -286,6 +292,17 @@ class Context:
                                                     C.byref(params), C.c_void_p(device_ptr), 1 if sync else 0),
                     "lt_render_views_device")
 
+    def render_masked_device(self, scene, camera, params, out_ptr, mask_ptr=None, m2_ptr=None, sync=False):
+        """lt_render_masked_device: lt_render_device for the pixels whose byte of the H x W uint8 mask at mask_ptr is
+        nonzero (None: every pixel); pixels outside the mask are not written.  m2_ptr: H * W * 3 floats of Welford sums
+        beside a running mean (None: not kept).  All pointers are device memory of the context's device, e.g. torch
+        CUDA tensors' data_ptr()."""
+        cam = np.ascontiguousarray(camera, dtype=L.CAMERA)
+        self._check(self.lib.lt_render_masked_device(self.h, scene.h, cam.ctypes.data, C.byref(params),
+                                                     C.c_void_p(mask_ptr) if mask_ptr else None, C.c_void_p(out_ptr),
+                                                     C.c_void_p(m2_ptr) if m2_ptr else None, 1 if sync else 0),
+                    "lt_render_masked_device")
+
     def accum_reset(self):
         self._check(self.lib.lt_accum_reset(self.h), "lt_accum_reset")
 
@@ -377,6 +394,11 @@ class Context:
         device-built copies); deterministic launches on scenes of at least stream_min_nodes nodes run k_flat_stream."""
         self._check(self.lib.lt_debug_ctx_limits(self.h, threaded_max_nodes, stream_min_nodes), "lt_debug_ctx_limits")
 
+    def debug_list_order(self, reversed):
+        """Test hook: later render_masked_device calls render their pixel list in reverse order (reversed=True) or in
+        the compaction's order (False, the default); the output is the same either way."""
+        self._check(self.lib.lt_debug_ctx_list_order(self.h, 1 if reversed else 0), "lt_debug_ctx_list_order")
+
     def stats(self):
         s = Stats()
         self.lib.lt_last_stats(self.h, C.byref(s))
@@ -432,6 +454,20 @@ def plan_views(params, view_count, node_count, stack_depth, total_mem, sm_count)
     rc = lib.lt_debug_plan_views(C.byref(params), view_count, node_count, stack_depth, total_mem, sm_count, out)
     if rc == ERR_INVALID:
         raise LtError("lt_debug_plan_views failed (%d): %s" % (rc, lib.lt_last_error(None).decode()))
+    d = dict(zip(PLAN_FIELDS, out))
+    d["error"] = rc
+    d["message"] = lib.lt_last_error(None).decode() if rc else ""
+    return d
+
+
+def plan_masked(params, pixel_count, node_count, stack_depth, total_mem, sm_count):
+    """Host-only: the launch plan of an lt_render_masked_device call whose mask lists pixel_count pixels
+    (lt_debug_plan_masked), as plan()."""
+    lib = load()
+    out = (C.c_int64 * len(PLAN_FIELDS))()
+    rc = lib.lt_debug_plan_masked(C.byref(params), pixel_count, node_count, stack_depth, total_mem, sm_count, out)
+    if rc == ERR_INVALID:
+        raise LtError("lt_debug_plan_masked failed (%d): %s" % (rc, lib.lt_last_error(None).decode()))
     d = dict(zip(PLAN_FIELDS, out))
     d["error"] = rc
     d["message"] = lib.lt_last_error(None).decode() if rc else ""

@@ -214,6 +214,7 @@ extern "C" void lt_ctx_destroy(lt_ctx* ctx) {
   if (ctx->dSample) cudaFree(ctx->dSample);
   if (ctx->dViews) cudaFree(ctx->dViews);
   if (ctx->dViewFrameCounts) cudaFree(ctx->dViewFrameCounts);
+  if (ctx->dMaskList) cudaFree(ctx->dMaskList);
   delete ctx->copyPool;
   if (ctx->stage) cudaFreeHost(ctx->stage);
   for (cudaEvent_t e : ctx->stageEvents) cudaEventDestroy(e);
@@ -568,6 +569,19 @@ static LtSceneDev scene_for_plan(const lt_scene* s, const LtPlan& plan) {
   return d;
 }
 
+// Is p memory of the context's device (device or managed memory), aligned to `align` bytes?  Fails with LT_ERR_INVALID
+// naming `what` otherwise.
+static int check_device_memory(lt_ctx* ctx, const void* p, size_t align, const std::string& w, const char* what) {
+  cudaPointerAttributes pa;
+  if (cudaPointerGetAttributes(&pa, p) != cudaSuccess ||
+      (pa.type != cudaMemoryTypeDevice && pa.type != cudaMemoryTypeManaged) || pa.device != ctx->device) {
+    cudaGetLastError();
+    return fail(ctx, LT_ERR_INVALID, w + what + " is not device memory of the context's device");
+  }
+  if ((uintptr_t)p % align) return fail(ctx, LT_ERR_INVALID, w + what + " is not " + std::to_string(align) + "-byte aligned");
+  return LT_OK;
+}
+
 // Both forms of lt_scene_refit, after the checks that need no device: `src` holds the scene's primitive count of new
 // primitives in host memory, already checked, or in device memory (onDevice), checked here by a kernel.  Nothing of
 // the scene is written before every check has passed.  The topology's parents and inner-node ranks are derived on the
@@ -577,16 +591,8 @@ static int refit_scene(lt_ctx* ctx, lt_scene* s, const void* src, bool onDevice,
   CK(cudaSetDevice(ctx->device));
   const int n = s->dev.nodeCount, nPrims = s->dev.primCount;
   cudaStream_t st = ctx->stream;
-  if (onDevice) {
-    cudaPointerAttributes pa;
-    if (cudaPointerGetAttributes(&pa, src) != cudaSuccess ||
-        (pa.type != cudaMemoryTypeDevice && pa.type != cudaMemoryTypeManaged) || pa.device != ctx->device) {
-      cudaGetLastError();
-      return fail(ctx, LT_ERR_INVALID, w + "device_primitives is not device memory of the context's device");
-    }
-    if ((uintptr_t)src % alignof(RefPrim))
-      return fail(ctx, LT_ERR_INVALID, w + "device_primitives is not 4-byte aligned");
-  }
+  if (onDevice)
+    if (int rc = check_device_memory(ctx, src, alignof(RefPrim), w, "device_primitives")) return rc;
   // The upload checks only a leaf's first primitive (the reference's leaves test no other, SURVEY H1); the refit reads
   // all of them, so every leaf's range must lie in the primitive buffer.
   if (s->refitLeaves == 0) {
@@ -705,10 +711,13 @@ int lt_internal_ensure_out(lt_ctx* ctx, size_t floats) {
 }
 
 // cams: the cameras of a call of several views (viewCount >= 2, view v into dOut + v * W * H * depth); nullptr: L.cam
+// list: the listed pixels of a masked call (lt_render_masked_device), or nullptr
 static int render_common(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, float* dOut, bool sync,
-                         const RefCamera* cams = nullptr, int viewCount = 1) {
+                         const RefCamera* cams = nullptr, int viewCount = 1, const LtList* list = nullptr) {
   CK(cudaSetDevice(ctx->device));
-  LtPlan plan = lt_plan_render(L, scene_facts(scene), ctx->totalMem, ctx->stats.sm_count, ctx->limits, viewCount);
+  const long long listed = list ? list->count : -1;
+  LtPlan plan =
+      lt_plan_render(L, scene_facts(scene), ctx->totalMem, ctx->stats.sm_count, ctx->limits, viewCount, listed);
   if (plan.error != LT_OK) return fail(ctx, plan.error, plan.message);
   const bool stats = plan.stats;
   if (stats) CK(cudaMemsetAsync(ctx->dCounters, 0, sizeof(LtCounters), ctx->stream));
@@ -719,7 +728,7 @@ static int render_common(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, float*
     // not a fallback to other arithmetic: the megakernel is the same path per pixel
     LtLaunch mega = L;
     mega.flags |= LT_FLAG_MEGAKERNEL;
-    plan = lt_plan_render(mega, scene_facts(scene), ctx->totalMem, ctx->stats.sm_count, ctx->limits, viewCount);
+    plan = lt_plan_render(mega, scene_facts(scene), ctx->totalMem, ctx->stats.sm_count, ctx->limits, viewCount, listed);
   }
   const bool wavefront = plan.pipeline == LT_PIPE_WAVEFRONT;
   const int kMaxTracePairs = 8192;
@@ -750,7 +759,7 @@ static int render_common(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, float*
     launches = lt_launch_render_wavefront(sc, plan, L, dOut, ctx->dCounters, ctx->wfWorkspace, ctx->stats.sm_count,
                                           ctx->stream, timeTrace ? ctx->traceEvents.data() : nullptr, kMaxTracePairs,
                                           &tracePairs, timeKinds ? ctx->pairKinds.data() : nullptr, &ctx->wfAux,
-                                          viewCount > 1 ? &views : nullptr);
+                                          viewCount > 1 ? &views : nullptr, list);
   } else if (viewCount > 1) {  // the megakernels: one launch per view, back to back on the stream
     for (int v = 0; v < viewCount; v++) {
       LtLaunch Lv = L;
@@ -759,7 +768,7 @@ static int render_common(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, float*
                                    ctx->dWork, ctx->stream);
     }
   } else {
-    launches = lt_launch_render(sc, plan, L, dOut, ctx->dCounters, ctx->dWork, ctx->stream);
+    launches = lt_launch_render(sc, plan, L, dOut, ctx->dCounters, ctx->dWork, ctx->stream, list);
   }
   CK(cudaGetLastError());
   CK(cudaEventRecord(ctx->ev1, ctx->stream));
@@ -812,6 +821,61 @@ extern "C" int lt_render_device(lt_ctx* ctx, lt_scene* scene, const void* camera
   if (rc != LT_OK) return rc;
   if (!device_out) return fail(ctx, LT_ERR_INVALID, "lt_render_device: device_out is NULL");
   return render_common(ctx, scene, L, device_out, sync != 0);
+}
+
+// lt_render_masked_device: the pixel list in ctx->dMaskList, its count first, the list from kMaskListAt on (256 B)
+static const size_t kMaskListAt = 64;
+
+extern "C" int lt_render_masked_device(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params,
+                                       const uint8_t* device_mask, float* device_out, float* device_m2, int sync) {
+  const std::string w = "lt_render_masked_device: ";
+  if (ctx && ctx->group)
+    return fail(ctx, LT_ERR_UNSUPPORTED, w + "a multi-GPU context renders into host memory (lt_render)");
+  LtLaunch L;
+  if (int rc = check_params(ctx, scene, camera28, params, &L)) return rc;
+  if (!device_out) return fail(ctx, LT_ERR_INVALID, w + "device_out is NULL");
+  if (int rc = lt_masked_image_check(ctx, L, "lt_render_masked_device")) return rc;
+  if (device_m2 && (L.accumMode != LT_ACCUM_RUNNING_MEAN || L.frameStride > 1))
+    return fail(ctx, LT_ERR_INVALID, w + "device_m2 needs accum_mode LT_ACCUM_RUNNING_MEAN and frame_stride <= 1");
+  if (device_mask)
+    if (int rc = check_device_memory(ctx, device_mask, 1, w, "device_mask")) return rc;
+  if (device_m2)
+    if (int rc = check_device_memory(ctx, device_m2, alignof(float), w, "device_m2")) return rc;
+  CK(cudaSetDevice(ctx->device));
+  const size_t pixels = (size_t)L.width * L.height;
+  CK(ctx_grow(&ctx->dMaskList, &ctx->maskListSize, kMaskListAt + pixels, sizeof(int)));
+  int* dCount = ctx->dMaskList;
+  int* dList = ctx->dMaskList + kMaskListAt;
+  lt_launch_mask_compact(device_mask, L.width, L.height, dList, dCount, ctx->stream);
+  CK(cudaGetLastError());
+  // the plan sizes the launch by the listed pixels: their count comes back to the host (no mask: all of them)
+  int count = (int)pixels;
+  if (device_mask) {
+    CK(cudaMemcpyAsync(&count, dCount, sizeof count, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+  }
+  if (count == 0) {  // nothing to render: no pixel is written
+    const int sms = ctx->stats.sm_count;
+    const float uploadMs = ctx->stats.upload_ms;
+    ctx->stats = lt_stats{};
+    ctx->stats.sm_count = sms;
+    ctx->stats.upload_ms = uploadMs;
+    ctx->stats.kernel_launches = 1;
+    return LT_OK;
+  }
+  const int extra = ctx->reverseList ? lt_launch_list_reverse(dList, count, ctx->stream) : 0;
+  const LtList list = {dList, count, device_m2};
+  const int rc = render_common(ctx, scene, L, device_out, sync != 0, nullptr, 1, &list);
+  ctx->stats.kernel_launches += 1 + extra;  // the compaction (and the test hook's reversal)
+  return rc;
+}
+
+extern "C" int lt_debug_ctx_list_order(lt_ctx* ctx, int reversed) {
+  if (!ctx) return fail(nullptr, LT_ERR_INVALID, "lt_debug_ctx_list_order: ctx is NULL");
+  if (ctx->group) return fail(ctx, LT_ERR_UNSUPPORTED, "lt_debug_ctx_list_order: not available on a multi-GPU context");
+  if (reversed != 0 && reversed != 1) return fail(ctx, LT_ERR_INVALID, "lt_debug_ctx_list_order: reversed must be 0 or 1");
+  ctx->reverseList = reversed != 0;
+  return LT_OK;
 }
 
 int lt_internal_render_rows(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params,

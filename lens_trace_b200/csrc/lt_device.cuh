@@ -710,6 +710,56 @@ struct FrameSink {
   }
 };
 
+// Beside a running mean (lt_render_masked_device's m2): per channel, the sum of squared deviations of the frame samples
+// the mean averages (Welford), 3 floats per pixel at m2 + 3 * pixel.  A frame with frameCount n and sample x, the mean
+// before it `prev` and after it `mean` (FrameSink::frame): n == 0 restarts at 0, otherwise m2 += (x - prev) * (x - mean),
+// one rounding per operation.
+struct M2Sink {
+  float m2[3];
+  // loads what earlier frames left when the first frame of this launch continues them (frameCount > 0)
+  __device__ __forceinline__ void begin(bool load, const float* p, long long pixel) {
+    m2[0] = m2[1] = m2[2] = 0.0f;
+    if (load) {
+      m2[0] = p[3 * pixel + 0];
+      m2[1] = p[3 * pixel + 1];
+      m2[2] = p[3 * pixel + 2];
+    }
+  }
+  __device__ __forceinline__ void frame(unsigned n, const float x[3], const float prev[3], const float mean[3]) {
+#pragma unroll
+    for (int k = 0; k < 3; k++) m2[k] = n == 0u ? 0.0f : FADD(m2[k], FMUL(FSUB(x[k], prev[k]), FSUB(x[k], mean[k])));
+  }
+  __device__ __forceinline__ void end(float* p, long long pixel) const {
+    p[3 * pixel + 0] = m2[0];
+    p[3 * pixel + 1] = m2[1];
+    p[3 * pixel + 2] = m2[2];
+  }
+};
+
+// one frame through the frame combiner, and with M2 through the Welford sum beside it
+template <bool M2>
+__device__ __forceinline__ void sink_frame(FrameSink& sink, M2Sink& w, const LtLaunch& L, unsigned frameCount,
+                                           const float c[3]) {
+  if (M2) {
+    const float prev[3] = {sink.acc[0], sink.acc[1], sink.acc[2]};
+    sink.frame(L, frameCount, c);
+    w.frame(frameCount, c, prev, sink.acc);
+  } else {
+    sink.frame(L, frameCount, c);
+  }
+}
+
+// thread -> listed pixel of a masked launch (lt_render_masked_device): thread i of the grid takes list[i], i < count
+// (unsigned: a grid over up to 2^31 - 1 listed pixels has threads past INT_MAX)
+__device__ __forceinline__ bool thread_list_pixel(const int* list, int count, int width, int& px, int& py) {
+  const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= (unsigned)count) return false;
+  const int pixel = list[i];
+  py = pixel / width;
+  px = pixel - py * width;
+  return true;
+}
+
 __device__ __forceinline__ void flush_counters(LtCounters* g, const LtCounters& c) {
   if (g) {
     atomicAdd(&g->rays, c.rays);

@@ -45,6 +45,15 @@ struct LtLaunch {
   RefCamera cam;
 };
 
+// The pixels of a masked launch (lt_render_masked_device): `count` pixel indices (py * width + px) at `list`, in the
+// order thread_pixel gives pixels to threads; m2: the Welford sums beside the running mean (M2Sink), or nullptr.
+// The kernels' LIST / M2 variants read it; the others take it as an unused last argument.
+struct LtList {
+  const int* list;
+  int count;
+  float* m2;
+};
+
 struct LtCounters {
   unsigned long long rays, nodeTests, triTests;
 };

@@ -49,14 +49,18 @@ struct LtSceneFacts {
 };
 LtTree lt_plan_threaded_copies(int nNodes, size_t totalMem, const LtLimits& lim);
 LtPlan lt_plan_primary_hits(int flags, int width, int height, const LtSceneFacts& s);
+// listed >= 0: a masked launch (lt_render_masked_device) of that many listed pixels, planned for them instead of the
+// width x height image
 LtPlan lt_plan_render(const LtLaunch& L, const LtSceneFacts& s, size_t totalMem, int smCount, const LtLimits& lim,
-                      int views = 1);
+                      int views = 1, long long listed = -1);
 // The struct-size check of a caller's lt_render_params and its zero-filled copy at *P, which has the current
 // struct_size; `w` starts the error message ("lt_render: ")
 int lt_params_normalise(lt_ctx* ctx, const lt_render_params* params, const std::string& w, lt_render_params* P);
 // lt_render_params -> the launch descriptor (all of it but the camera), with lt_render's checks; `who` names the entry
 // point in error messages
 int lt_params_to_launch(lt_ctx* ctx, const lt_render_params* params, LtLaunch* L, const char* who = "lt_render");
+// LT_ERR_UNSUPPORTED (message set) for an image a masked call cannot number with 32-bit pixel indices
+int lt_masked_image_check(lt_ctx* ctx, const LtLaunch& L, const char* who);
 
 // ---- host tree builders (lt_tree.cpp) ----
 // Host-side validation of the reference node array (bounds of every index the kernels will follow) and the depth the
@@ -75,14 +79,19 @@ int lt_launch_build_threaded(const RefNode* dNodes, int nodeCount, LtThreadNode*
 size_t lt_scan_temp_bytes(int n);
 int lt_launch_exclusive_scan(void* dTemp, size_t tempBytes, const int* dIn, int* dOut, int n, cudaStream_t stream);
 // dWork: one zero-initialisable int of device memory (work counter of the persistent kernels)
+// list: the pixels of a masked launch (k_flat / k_path over the list, grid = plan.grid), or nullptr
 int lt_launch_render(const LtSceneDev& sc, const LtPlan& plan, const LtLaunch& L, float* dOut, LtCounters* dCounters,
-                     int* dWork, cudaStream_t stream);
+                     int* dWork, cudaStream_t stream, const LtList* list = nullptr);
+// the set pixels of a width x height byte mask (nullptr: all) -> dList, their number -> *dCount (k_mask_compact)
+int lt_launch_mask_compact(const unsigned char* dMask, int width, int height, int* dList, int* dCount,
+                           cudaStream_t stream);
+int lt_launch_list_reverse(int* dList, int count, cudaStream_t stream);  // the list in reverse order, in place
 int lt_launch_primary_hits(const LtSceneDev& sc, const LtPlan& plan, const RefCamera& cam, int kernel, int flags,
                            int width, int height, int* dIds, int* dHit, float* dTuv, cudaStream_t stream);
 // Dynamic shared memory beyond 48 KB needs an opt-in per kernel and device: given once for every traversal kernel
 // (both files), the first time a launch asks for more.
 void lt_opt_in_traversal_smem(size_t smem);
-extern const void* const lt_wf_traversal_kernels[7];  // lt_wavefront.cu
+extern const void* const lt_wf_traversal_kernels[10];  // lt_wavefront.cu
 int lt_launch_debug_random(const float* fx, const float* fy, const float* seed, int n, float* out, cudaStream_t stream);
 int lt_launch_debug_hemisphere(const float* u1, const float* u2, const float* up, int n, float* out,
                                cudaStream_t stream);
@@ -116,7 +125,8 @@ enum { LT_TIMED_TRAVERSAL = 0, LT_TIMED_SHADE = 1, LT_TIMED_PRIMARY_SHADE = 2, L
 int lt_launch_render_wavefront(const LtSceneDev& sc, const LtPlan& plan, const LtLaunch& L, float* dOut,
                                LtCounters* dCounters, void* workspace, int smCount, cudaStream_t stream,
                                cudaEvent_t* traceEvents, int maxTraceLaunches, int* traceLaunches,
-                               unsigned char* pairKinds, const LtWfAux* aux, const LtViews* views);
+                               unsigned char* pairKinds, const LtWfAux* aux, const LtViews* views,
+                               const LtList* list = nullptr);
 
 // user-written CUDA kernels with the reference's plug-in ABI (lt_plugin.cu)
 struct LtPlugin;
@@ -187,6 +197,9 @@ struct lt_ctx {
   size_t viewsFloats = 0;
   unsigned* dViewFrameCounts = nullptr;  // LtViews::dFrameCounts of a wavefront views launch
   size_t viewFrameCountsSize = 0;
+  int* dMaskList = nullptr;  // lt_render_masked_device: the listed pixels' count, then (from kMaskListAt) the list
+  size_t maskListSize = 0;
+  bool reverseList = false;  // lt_debug_ctx_list_order: masked calls render their list in reverse order
   size_t totalMem = 0;
   char* stage = nullptr;  // pinned staging buffer of lt_render's copy into a pageable destination
   size_t stageBytes = 0;

@@ -19,12 +19,13 @@
 
 #include <cub/device/device_scan.cuh>
 
-template <bool STATS>
+// LIST: thread i renders pixel M.list[i] (a masked launch); M2: and keeps the Welford sums at M.m2 (running mean only)
+template <bool STATS, bool LIST, bool M2>
 __global__ void __launch_bounds__(LT_BLOCK) k_flat(LtSceneDev sc, LtLaunch L, float* __restrict__ out,
-                                                   LtCounters* gcnt) {
+                                                   LtCounters* gcnt, LtList M) {
   LT_TRAV_SMEM(s, lt_stack_levels(sc))
   int px, py;
-  if (!thread_pixel(L.width, L.height, px, py)) return;
+  if (LIST ? !thread_list_pixel(M.list, M.count, L.width, px, py) : !thread_pixel(L.width, L.height, px, py)) return;
   LtCounters cnt = {0, 0, 0};
   float fx, fy;
   Trav t;
@@ -50,12 +51,16 @@ __global__ void __launch_bounds__(LT_BLOCK) k_flat(LtSceneDev sc, LtLaunch L, fl
       color[2] = mat->diffuse[2];
     }
   }
-  long long id = ((long long)py * L.width + px) * L.depth;
+  const long long pixel = (long long)py * L.width + px;
+  long long id = pixel * L.depth;
   FrameSink sink;
   sink.begin(L, out, id);
+  M2Sink w;
+  if (M2) w.begin(L.cam.frameCount > 0, M.m2, pixel);
   // the image is the same for every frame (no RNG): apply the frame combiner `frames` times
-  for (int f = 0; f < L.frames; f++) sink.frame(L, L.cam.frameCount + (unsigned)f * L.frameStride, color);
+  for (int f = 0; f < L.frames; f++) sink_frame<M2>(sink, w, L, L.cam.frameCount + (unsigned)f * L.frameStride, color);
   sink.end(out, id);
+  if (M2) w.end(M.m2, pixel);
   if (STATS) {
     cnt.rays *= (unsigned)L.frames;
     cnt.nodeTests *= (unsigned)L.frames;
@@ -145,13 +150,14 @@ __global__ void __launch_bounds__(LT_BLOCK) k_flat_stream(LtSceneDev sc, LtLaunc
 //     waiting for a new ray, so long rays never hold the other 31 lanes idle.  Traversal state is
 //     resumable.
 constexpr int kPathRefillLanes = 4;
-template <bool STATS>
+// LIST, M2: as k_flat
+template <bool STATS, bool LIST, bool M2>
 __global__ void __launch_bounds__(LT_BLOCK) k_path(LtSceneDev sc, LtLaunch L, float* __restrict__ out,
-                                                   LtCounters* gcnt) {
+                                                   LtCounters* gcnt, LtList M) {
   // the persistent megakernel does not cull (LT_FLAG_CULL selects the wavefront pipeline)
   LT_TRAV_SMEM(s, lt_stack_levels(sc))
   int px, py;
-  bool alive = thread_pixel(L.width, L.height, px, py);
+  bool alive = LIST ? thread_list_pixel(M.list, M.count, L.width, px, py) : thread_pixel(L.width, L.height, px, py);
   LtCounters cnt = {0, 0, 0};
   const PathConsts pc = path_consts(L);
 
@@ -160,10 +166,13 @@ __global__ void __launch_bounds__(LT_BLOCK) k_path(LtSceneDev sc, LtLaunch L, fl
   long long id = 0;
   FrameSink sink;
   sink.acc[0] = sink.acc[1] = sink.acc[2] = 0.0f;
+  M2Sink w;
+  if (M2) w.m2[0] = w.m2[1] = w.m2[2] = 0.0f;
   if (alive) {
     cameraRay = camera_ray(L.cam, px, lt_image_row(L, py), L.width, L.fullHeight, fx, fy);
     id = ((long long)py * L.width + px) * L.depth;
     sink.begin(L, out, id);
+    if (M2) w.begin(L.cam.frameCount > 0, M.m2, (long long)py * L.width + px);
   }
 
   int frame = 0, sample = 0;
@@ -201,11 +210,12 @@ __global__ void __launch_bounds__(LT_BLOCK) k_path(LtSceneDev sc, LtLaunch L, fl
         sample++;
         if (sample == pc.samplesPerFrame) {
           finish_frame_colour(pc, L.kernelMode, frameColor);
-          sink.frame(L, L.cam.frameCount + (unsigned)frame * L.frameStride, frameColor);
+          sink_frame<M2>(sink, w, L, L.cam.frameCount + (unsigned)frame * L.frameStride, frameColor);
           sample = 0;
           frame++;
           if (frame >= L.frames) {
             sink.end(out, id);
+            if (M2) w.end(M.m2, id / L.depth);
             alive = false;
             break;
           }
@@ -392,9 +402,50 @@ __global__ void k_plugin_accumulate(LtLaunch L, const float* __restrict__ sample
   }
 }
 
+// The pixels of a mask (nonzero bytes, width x height row-major; nullptr: every pixel) as the pixel list of a masked
+// launch: thread t of a full-image grid looks at the pixel thread_pixel gives it, and each warp appends its set pixels
+// in lane order with one atomic, so a warp's 8x4 tile stays together in the list and the camera rays of the threads
+// that render it stay coherent.  The order of the warps' runs varies from call to call; no pixel's value depends on it.
+__global__ void __launch_bounds__(LT_BLOCK) k_mask_compact(const unsigned char* __restrict__ mask, int width,
+                                                           int height, int* __restrict__ list, int* __restrict__ count) {
+  int px, py;
+  const bool valid = thread_pixel(width, height, px, py);
+  const int pixel = valid ? py * width + px : 0;
+  const bool set = valid && (mask == nullptr || mask[pixel] != 0);
+  const unsigned lane = threadIdx.x & 31u, m = __ballot_sync(0xffffffffu, set);
+  if (m == 0u) return;
+  int base = 0;
+  if (lane == 0u) base = atomicAdd(count, __popc(m));
+  base = __shfl_sync(0xffffffffu, base, 0);
+  if (set) list[base + __popc(m & ((1u << lane) - 1u))] = pixel;
+}
+
+// lt_debug_ctx_list_order: the list of a masked launch in reverse order, so that tests can render one mask through two
+// list orders
+__global__ void k_list_reverse(int* __restrict__ list, int count) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= count / 2) return;
+  const int a = list[i], b = list[count - 1 - i];
+  list[i] = b;
+  list[count - 1 - i] = a;
+}
+
 // ------------------------------------------------------------------------------------------------
 // host-side launchers
 // ------------------------------------------------------------------------------------------------
+int lt_launch_list_reverse(int* dList, int count, cudaStream_t stream) {
+  if (count < 2) return 0;
+  k_list_reverse<<<(count / 2 + 255) / 256, 256, 0, stream>>>(dList, count);
+  return 1;
+}
+
+int lt_launch_mask_compact(const unsigned char* dMask, int width, int height, int* dList, int* dCount,
+                           cudaStream_t stream) {
+  cudaMemsetAsync(dCount, 0, sizeof(int), stream);
+  k_mask_compact<<<((width + 15) / 16) * ((height + 7) / 8), LT_BLOCK, 0, stream>>>(dMask, width, height, dList, dCount);
+  return 1;
+}
+
 int lt_launch_debug_random(const float* fx, const float* fy, const float* seed, int n, float* out, cudaStream_t stream) {
   k_debug_random<<<(n + 255) / 256, 256, 0, stream>>>(fx, fy, seed, n, out);
   return 1;
@@ -445,26 +496,43 @@ void lt_opt_in_traversal_smem(size_t smem) {
   cudaGetDevice(&dev);
   if (dev < 0 || dev >= 64 || done[dev]) return;
   done[dev] = true;
-  const void* const mine[] = {(const void*)k_flat<false>, (const void*)k_flat<true>, (const void*)k_path<false>,
-                              (const void*)k_path<true>, (const void*)k_primary_hits, (const void*)k_flat_stream};
+  const void* const mine[] = {(const void*)k_flat<false, false, false>, (const void*)k_flat<true, false, false>,
+                              (const void*)k_flat<false, true, false>,  (const void*)k_flat<true, true, false>,
+                              (const void*)k_flat<false, true, true>,   (const void*)k_flat<true, true, true>,
+                              (const void*)k_path<false, false, false>, (const void*)k_path<true, false, false>,
+                              (const void*)k_path<false, true, false>,  (const void*)k_path<true, true, false>,
+                              (const void*)k_path<false, true, true>,   (const void*)k_path<true, true, true>,
+                              (const void*)k_primary_hits,              (const void*)k_flat_stream};
   for (const void* k : mine) cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxTraversalSmem);
   for (const void* k : lt_wf_traversal_kernels)
     cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxTraversalSmem);
 }
 
-int lt_launch_render(const LtSceneDev& sc, const LtPlan& plan, const LtLaunch& L, float* dOut, LtCounters* dCounters,
-                     int* dWork, cudaStream_t stream) {
-  lt_opt_in_traversal_smem(plan.smemStack);
+template <bool LIST, bool M2>
+static void launch_megakernel(const LtSceneDev& sc, const LtPlan& plan, const LtLaunch& L, float* dOut,
+                              LtCounters* dCounters, const LtList& M, cudaStream_t stream) {
   const size_t smem = plan.smemStack;
+  if (plan.pipeline == LT_PIPE_FLAT) {
+    if (plan.stats) k_flat<true, LIST, M2><<<plan.grid, LT_BLOCK, smem, stream>>>(sc, L, dOut, dCounters, M);
+    else k_flat<false, LIST, M2><<<plan.grid, LT_BLOCK, smem, stream>>>(sc, L, dOut, nullptr, M);
+  } else {
+    if (plan.stats) k_path<true, LIST, M2><<<plan.grid, LT_BLOCK, smem, stream>>>(sc, L, dOut, dCounters, M);
+    else k_path<false, LIST, M2><<<plan.grid, LT_BLOCK, smem, stream>>>(sc, L, dOut, nullptr, M);
+  }
+}
+
+int lt_launch_render(const LtSceneDev& sc, const LtPlan& plan, const LtLaunch& L, float* dOut, LtCounters* dCounters,
+                     int* dWork, cudaStream_t stream, const LtList* list) {
+  lt_opt_in_traversal_smem(plan.smemStack);
   if (plan.pipeline == LT_PIPE_FLAT_STREAM) {
     cudaMemsetAsync(dWork, 0, sizeof(int), stream);
-    k_flat_stream<<<plan.grid, LT_BLOCK, smem, stream>>>(sc, L, dOut, dWork);
-  } else if (plan.pipeline == LT_PIPE_FLAT) {
-    if (plan.stats) k_flat<true><<<plan.grid, LT_BLOCK, smem, stream>>>(sc, L, dOut, dCounters);
-    else k_flat<false><<<plan.grid, LT_BLOCK, smem, stream>>>(sc, L, dOut, nullptr);
+    k_flat_stream<<<plan.grid, LT_BLOCK, plan.smemStack, stream>>>(sc, L, dOut, dWork);
+  } else if (!list) {
+    launch_megakernel<false, false>(sc, plan, L, dOut, dCounters, LtList{}, stream);
+  } else if (!list->m2) {
+    launch_megakernel<true, false>(sc, plan, L, dOut, dCounters, *list, stream);
   } else {
-    if (plan.stats) k_path<true><<<plan.grid, LT_BLOCK, smem, stream>>>(sc, L, dOut, dCounters);
-    else k_path<false><<<plan.grid, LT_BLOCK, smem, stream>>>(sc, L, dOut, nullptr);
+    launch_megakernel<true, true>(sc, plan, L, dOut, dCounters, *list, stream);
   }
   return 1;
 }

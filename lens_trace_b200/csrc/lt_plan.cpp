@@ -4,6 +4,7 @@
 #include "lens_trace_b200.h"
 #include "lt_internal.h"
 
+#include <limits.h>
 #include <stddef.h>
 #include <string.h>
 
@@ -63,15 +64,31 @@ LtPlan lt_plan_primary_hits(int flags, int width, int height, const LtSceneFacts
 // The lighting kernels keep their factor of 4 (not measured for views).
 static const long long kViewsMinPaths = 3ll << 20;
 
+// A masked call's list of scattered pixels (lt_render_masked_device with a partial mask) gives the megakernel no
+// coherent camera rays, and its blocks wait for their longest thread over all frames.  Measured (tools/masked_timing.py,
+// profiles/masked_timing_b200.txt; NVIDIA B200 at its 1000 W power limit): GI, 4 bounces, Cornell box, random masks of
+// a 1080p image, ms of the megakernel against the wavefront: N = 2^12 .. 2^20 pixels at 1 frame 0.155 / 0.456 ..
+// 0.869 / 0.760, at 4 frames 0.430 / 0.597 (2^12), 0.480 / 0.652 (2^16), 1.004 / 0.792 (2^18), at 16 frames
+// 1.451 / 0.618 (2^12) .. 11.86 / 3.50 (2^20); a quarter of the image, 16 frames, 6.49 / 2.04, on the 1 M-triangle
+// mesh 43.1 / 12.6.  So GI lists take the wavefront from 2^20 paths, and from 2^16 paths at 16 or more frames.
+static const long long kMaskedMinPaths = 1ll << 20, kMaskedManyFramesMinPaths = 1ll << 16;
+static const int kMaskedManyFrames = 16;
+
 // views: a call of several views (lt_render_views) runs its (view, frame) pairs through one wavefront launch, or one
 // megakernel launch per view
+// listed >= 0: a masked call (lt_render_masked_device) renders that many listed pixels; every size below counts them
+// where an unmasked call counts the image's pixels (the wavefront's threshold, frames per batch, the 2^25 paths per
+// frame, its workspace and records, the grids), so a full mask plans as the unmasked call.  A partial GI list also
+// takes the wavefront at the lower thresholds measured for scattered pixels (kMaskedMinPaths).  The deterministic
+// kernels run k_flat over the list: k_flat_stream fetches whole 8x4 tiles (same output either way).
 LtPlan lt_plan_render(const LtLaunch& L, const LtSceneFacts& s, size_t totalMem, int smCount, const LtLimits& lim,
-                      int views) {
+                      int views, long long listed) {
   LtPlan p = {};
   p.error = LT_OK;
   p.stats = (L.flags & LT_FLAG_STATS) != 0;
   p.cull = (L.flags & LT_FLAG_CULL) != 0;
-  const long long pixels = (long long)L.width * L.height;
+  const bool masked = listed >= 0;
+  const long long pixels = masked ? listed : (long long)L.width * L.height;
   const bool isGI = L.kernel == LT_KERNEL_GI25 || L.kernel == LT_KERNEL_GI;
   // stochastic kernels: wavefront pipeline for large launches, persistent megakernel for small ones
   p.pipeline = L.kernel >= LT_KERNEL_LIGHTING25 ? LT_PIPE_PATH : LT_PIPE_FLAT;
@@ -86,6 +103,11 @@ LtPlan lt_plan_render(const LtLaunch& L, const LtSceneFacts& s, size_t totalMem,
     const long long pairs = (long long)L.frames * views;  // (view, frame) pairs, view-major
     bool wavefront = forced || (pixels * pairs >= need && L.kernel != LT_KERNEL_GI25 &&
                                 L.kernel != LT_KERNEL_LIGHTING25);
+    // a partial list (a full one plans as the image): the measured thresholds of scattered pixels above
+    if (masked && pixels < (long long)L.width * L.height && L.kernel == LT_KERNEL_GI &&
+        (pixels * pairs >= kMaskedMinPaths ||
+         (L.frames >= kMaskedManyFrames && pixels * pairs >= kMaskedManyFramesMinPaths)))
+      wavefront = true;
     // A queue entry carries the bounce depth in 5 bits (wf_pack_path): deeper bounce caps stay on the megakernel,
     // which is the same arithmetic per path (0 = the reference constant 16).  It carries its path id in 25 bits:
     // one frame must fit.
@@ -143,7 +165,7 @@ LtPlan lt_plan_render(const LtLaunch& L, const LtSceneFacts& s, size_t totalMem,
   if (p.blocksPerSm > 8) p.blocksPerSm = 8;
   if (p.blocksPerSm < 1) p.blocksPerSm = 1;
   // exact, uncounted launches of the deterministic pipelines on large scenes: persistent warps fetching tiles
-  if (p.pipeline == LT_PIPE_FLAT && !(L.flags & (LT_FLAG_STATS | LT_FLAG_CULL | LT_FLAG_NO_STREAM)) &&
+  if (p.pipeline == LT_PIPE_FLAT && !masked && !(L.flags & (LT_FLAG_STATS | LT_FLAG_CULL | LT_FLAG_NO_STREAM)) &&
       p.tree == LT_TREE_CHILD_PAIR && s.nodeCount >= lim.streamMinNodes)
     p.pipeline = LT_PIPE_FLAT_STREAM;
   if (p.pipeline == LT_PIPE_FLAT_STREAM) {
@@ -151,8 +173,10 @@ LtPlan lt_plan_render(const LtLaunch& L, const LtSceneFacts& s, size_t totalMem,
     p.grid = smCount * p.blocksPerSm < warpsNeeded ? smCount * p.blocksPerSm : warpsNeeded;
   } else if (p.pipeline == LT_PIPE_WAVEFRONT) {
     p.grid = smCount * p.blocksPerSm;
+  } else if (masked && pixels != (long long)L.width * L.height) {
+    p.grid = (int)((pixels + LT_BLOCK - 1) / LT_BLOCK);  // one thread per listed pixel
   } else {
-    p.grid = tile_blocks(L.width, L.height);
+    p.grid = tile_blocks(L.width, L.height);  // (a full list: the blocks of the unmasked launch, the last ones idle)
   }
   return p;
 }
@@ -201,15 +225,28 @@ int lt_params_to_launch(lt_ctx* ctx, const lt_render_params* params, LtLaunch* L
   return LT_OK;
 }
 
+// A masked call numbers the image's pixels, the listed ones and its list slots with 32-bit ints: images of more than
+// INT_MAX pixels are refused (lt_render_device renders them on the megakernels, which index with 64 bits)
+int lt_masked_image_check(lt_ctx* ctx, const LtLaunch& L, const char* who) {
+  if ((long long)L.width * L.height > (long long)INT_MAX)
+    return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED,
+                            std::string(who) + ": a masked call handles at most 2^31 - 1 pixels (width * height)");
+  return LT_OK;
+}
+
 static int debug_plan(const char* who, const lt_render_params* params, int views, uint64_t node_count,
-                      int32_t stack_depth, uint64_t total_mem, int32_t sm_count, int64_t* out) {
+                      int32_t stack_depth, uint64_t total_mem, int32_t sm_count, int64_t* out, long long listed = -1) {
   if (!params || !out || views < 1 || node_count < 1 || node_count > 0x7fffffffull || sm_count < 1)
     return lt_internal_fail(nullptr, LT_ERR_INVALID, std::string(who) + ": bad arguments");
   LtLaunch L = {};
   if (int rc = lt_params_to_launch(nullptr, params, &L)) return rc;
+  if (listed >= 0)
+    if (int rc = lt_masked_image_check(nullptr, L, who)) return rc;
+  if (listed >= 0 && (listed < 1 || listed > (long long)L.width * L.height))
+    return lt_internal_fail(nullptr, LT_ERR_INVALID, std::string(who) + ": pixel_count must be in [1, width * height]");
   const LtLimits lim;
   const LtSceneFacts s = {(int)node_count, stack_depth, lt_plan_threaded_copies((int)node_count, total_mem, lim)};
-  const LtPlan p = lt_plan_render(L, s, total_mem, sm_count, lim, views);
+  const LtPlan p = lt_plan_render(L, s, total_mem, sm_count, lim, views, listed);
   const int64_t v[LT_PLAN_FIELDS] = {p.pipeline, p.tree, p.stats, p.cull, p.batchFrames, p.streams, p.rounds,
                                      p.samplesPerFrame, p.sharedPrimary, p.classify, (int64_t)p.smemStack,
                                      (int64_t)p.smemTrace, p.blocksPerSm, p.grid, (int64_t)p.workspaceBytes};
@@ -225,4 +262,10 @@ extern "C" int lt_debug_plan(const lt_render_params* params, uint64_t node_count
 extern "C" int lt_debug_plan_views(const lt_render_params* params, int view_count, uint64_t node_count,
                                    int32_t stack_depth, uint64_t total_mem, int32_t sm_count, int64_t* out) {
   return debug_plan("lt_debug_plan_views", params, view_count, node_count, stack_depth, total_mem, sm_count, out);
+}
+
+extern "C" int lt_debug_plan_masked(const lt_render_params* params, int64_t pixel_count, uint64_t node_count,
+                                    int32_t stack_depth, uint64_t total_mem, int32_t sm_count, int64_t* out) {
+  return debug_plan("lt_debug_plan_masked", params, 1, node_count, stack_depth, total_mem, sm_count, out,
+                    pixel_count < 1 ? 0 : pixel_count);
 }

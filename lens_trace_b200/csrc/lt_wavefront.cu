@@ -79,9 +79,13 @@ __device__ __forceinline__ void wf_hit_unpack(int word, Hit& h) {
   h.hit = (int)((unsigned)word >> 31);
 }
 
-__device__ __forceinline__ void pixel_of_path(long long path, int pixels, int width, int& px, int& py, int& frameLocal) {
+// In a masked launch (LIST) the pixel axis of the path ids is the list index: path id = frame * count + i, pixel list[i]
+template <bool LIST = false>
+__device__ __forceinline__ void pixel_of_path(long long path, int pixels, int width, int& px, int& py, int& frameLocal,
+                                              const int* list = nullptr) {
   frameLocal = (int)(path / pixels);
   int pixel = (int)(path - (long long)frameLocal * pixels);
+  if (LIST) pixel = list[pixel];
   py = pixel / width;
   px = pixel - py * width;
 }
@@ -237,14 +241,18 @@ __device__ __forceinline__ void film_of_path(const LtWfPrimary& P, long long pat
   }
 }
 
+// LIST: a masked launch; `pixels` counts the listed pixels, and thread i traces pixel M.list[i] and writes its records
+// at i, so that the alive list holds list indices
+template <bool LIST>
 __global__ void __launch_bounds__(WF_BLOCK) k_wf_primary_trace(LtSceneDev sc, LtLaunch L, LtWfPrimary P, int pixels,
-                                                               int classify) {
+                                                               int classify, LtList M) {
   LT_TRAV_SMEM(s, lt_stack_levels(sc))
   const int pixel = blockIdx.x * blockDim.x + threadIdx.x;
   const bool valid = pixel < pixels;
   bool alive = false;
   if (valid) {
-    int py = pixel / L.width, px = pixel - py * L.width;
+    const int image = LIST ? M.list[pixel] : pixel;
+    int py = image / L.width, px = image - py * L.width;
     float fx, fy;
     Trav t;
     t.r = camera_ray(L.cam, px, lt_image_row(L, py), L.width, L.fullHeight, fx, fy);
@@ -277,10 +285,11 @@ __global__ void __launch_bounds__(WF_BLOCK) k_wf_primary_trace(LtSceneDev sc, Lt
 // out: the kind of round 1 (WF_FIRST_SHADOW, or WF_GENERIC), which decides what its entries hold
 // VIEWS: the nf frames are one view's frames inside a batch that holds several views (L.cam is that view's camera, P
 // its records); their paths are numbered from pathBase in the batch
-template <bool STATS, bool VIEWS>
+// LIST: a masked launch (`pixels` listed pixels); a launch that traces its camera rays here finds their pixels in M.list
+template <bool STATS, bool VIEWS, bool LIST>
 __global__ void __launch_bounds__(WF_BLOCK) k_wf_primary(LtSceneDev sc, LtLaunch L, LtWfBuffers B, int nf,
                                                          int pixels, int sample, LtCounters* gcnt, LtWfPrimary P,
-                                                         int out, int pathBase) {
+                                                         int out, int pathBase, LtList M) {
   LT_TRAV_SMEM(s, lt_stack_levels(sc))
   const float4* __restrict__ primaryHits = P.hits;
   const bool cull = (L.flags & LT_DEV_FLAG_CULL) != 0;  // closest-hit rays skip subtrees behind the current hit
@@ -316,7 +325,7 @@ __global__ void __launch_bounds__(WF_BLOCK) k_wf_primary(LtSceneDev sc, LtLaunch
         t.r.dx = t.r.dy = 0.0f;
         t.r.dz = 1.0f;
       } else {
-        pixel_of_path(p, pixels, L.width, px, py, fl);
+        pixel_of_path<LIST>(p, pixels, L.width, px, py, fl, M.list);
         t.r = camera_ray(L.cam, px, lt_image_row(L, py), L.width, L.fullHeight, fx, fy);
         if (cull) trace_cull<STATS>(t, sc, -1, pc.tInit, pc.epsThr, s, cnt);
         else trace<STATS>(t, sc, -1, pc.tInit, pc.epsThr, false, s, cnt);
@@ -552,27 +561,43 @@ __global__ void k_wf_swap(LtWfBuffers B, int q) {
 }
 
 // frames of the batch, in order, through the frame combiner (accumulator.frag:10-19)
+// LIST: a masked launch, thread i folds the frames of list index i into pixel M.list[i]; M2: and its Welford sums
+template <bool LIST, bool M2>
 __global__ void __launch_bounds__(WF_BLOCK) k_wf_accumulate(LtLaunch L, LtWfBuffers B, float* __restrict__ out,
                                                             int pixels, int frame0, int batchFrames,
-                                                            const unsigned char* __restrict__ cls) {
+                                                            const unsigned char* __restrict__ cls, LtList M) {
   const PathConsts pc = path_consts(L);
   int pixel = blockIdx.x * blockDim.x + threadIdx.x;
   if (pixel >= pixels) return;
-  long long id = (long long)pixel * L.depth;
+  const long long image = LIST ? M.list[pixel] : pixel;
+  long long id = image * L.depth;
   FrameSink sink;  // a batch that starts at frame0 > 0 continues from what earlier batches wrote to `out`
   if (frame0 == 0) sink.begin(L, out, id);
   else {
     sink.acc[0] = out[id + 0]; sink.acc[1] = out[id + 1]; sink.acc[2] = out[id + 2];
   }
+  M2Sink w;
+  if (M2) w.begin(frame0 > 0 || L.cam.frameCount > 0, M.m2, image);
   const int pixelClass = cls ? cls[pixel] : 2;  // black / white pixels have no paths: their sample is constant
   for (int f = 0; f < batchFrames; f++) {
     float4 v = make_float4((float)pixelClass, (float)pixelClass, (float)pixelClass, 0.0f);
     if (pixelClass == 2) v = B.frameCol[(long long)f * pixels + pixel];
     float c[3] = {v.x, v.y, v.z};
     finish_frame_colour(pc, L.kernelMode, c);
-    sink.frame(L, L.cam.frameCount + (unsigned)(frame0 + f) * L.frameStride, c);
+    sink_frame<M2>(sink, w, L, L.cam.frameCount + (unsigned)(frame0 + f) * L.frameStride, c);
   }
   sink.end(out, id);
+  if (M2) w.end(M.m2, image);
+}
+
+// The film table of a masked launch whose camera rays k_wf_primary traces itself (counting or culled launches): the
+// film position camera_ray computes for list index i, so that the shade kernels read it as in the other launches
+__global__ void __launch_bounds__(WF_BLOCK) k_wf_list_film(LtLaunch L, float2* __restrict__ film, LtList M) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= M.count) return;
+  const int pixel = M.list[i], py = pixel / L.width, px = pixel - py * L.width;
+  film[i] = make_float2(FADD(FDIV((float)px, (float)L.width), -0.5f),
+                        FADD(FDIV((float)lt_image_row(L, py), (float)L.fullHeight), -0.5f));
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -635,10 +660,12 @@ size_t lt_wf_view_records_bytes(long long pixels, int viewsPerBatch) {
 }
 
 // the kernels whose shared memory grows with the stack depth (lt_opt_in_traversal_smem)
-const void* const lt_wf_traversal_kernels[7] = {
-    (const void*)k_wf_primary_trace,      (const void*)k_wf_primary<false, false>, (const void*)k_wf_primary<true, false>,
-    (const void*)k_wf_primary<false, true>, (const void*)k_wf_primary<true, true>,   (const void*)k_wf_trace<false, false>,
-    (const void*)k_wf_trace<true, false>};
+const void* const lt_wf_traversal_kernels[10] = {
+    (const void*)k_wf_primary_trace<false>,        (const void*)k_wf_primary_trace<true>,
+    (const void*)k_wf_primary<false, false, false>, (const void*)k_wf_primary<true, false, false>,
+    (const void*)k_wf_primary<false, true, false>,  (const void*)k_wf_primary<true, true, false>,
+    (const void*)k_wf_primary<false, false, true>,  (const void*)k_wf_primary<true, false, true>,
+    (const void*)k_wf_trace<false, false>,          (const void*)k_wf_trace<true, false>};
 
 // Round r >= 1 of a sample (WfRound).  The exact pipelines fold the retracing of a light hit into its shading, so round
 // 1 holds the first shadow rays of the paths, and after it extension and shadow rounds alternate: an extension result
@@ -683,7 +710,8 @@ static int batch_segments(long long pair0, int nf, int frames, WfSegment* seg) {
 int lt_launch_render_wavefront(const LtSceneDev& sc, const LtPlan& plan, const LtLaunch& L, float* dOut,
                                LtCounters* dCounters, void* workspace, int smCount, cudaStream_t stream,
                                cudaEvent_t* traceEvents, int maxTraceLaunches, int* traceLaunches,
-                               unsigned char* pairKinds, const LtWfAux* aux, const LtViews* views) {
+                               unsigned char* pairKinds, const LtWfAux* aux, const LtViews* views,
+                               const LtList* list) {
   int pairs = 0;
   // which: 0 = before, 1 = after a launch; kind (LT_TIMED_*): what the bracketed kernel does.  Traversal launches
   // are always bracketed when events are given, the other kinds only when the caller passes pairKinds.
@@ -697,7 +725,9 @@ int lt_launch_render_wavefront(const LtSceneDev& sc, const LtPlan& plan, const L
     }
   };
   lt_opt_in_traversal_smem(plan.smemStack);
-  const int pixels = L.width * L.height;
+  // a masked launch (list): the pixel axis is the list index, `pixels` the listed pixels (views are not masked)
+  const int pixels = list ? list->count : L.width * L.height;
+  const LtList M = list ? *list : LtList{};
   const bool stats = plan.stats, threaded = plan.tree != LT_TREE_CHILD_PAIR, overlap = plan.streams == 2;
   const int batchFrames = plan.batchFrames;
   const size_t smem = plan.smemStack;
@@ -737,8 +767,12 @@ int lt_launch_render_wavefront(const LtSceneDev& sc, const LtPlan& plan, const L
   auto trace_primary = [&](const LtLaunch& Lv, const LtWfPrimary& P, cudaStream_t st) {
     if (plan.classify) cudaMemsetAsync(P.aliveCount, 0, sizeof(int), st);
     mark(0, st);
-    k_wf_primary_trace<<<(pixels + WF_BLOCK - 1) / WF_BLOCK, WF_BLOCK, smem, st>>>(sc, Lv, P, pixels,
-                                                                                  plan.classify ? 1 : 0);
+    if (list)
+      k_wf_primary_trace<true><<<(pixels + WF_BLOCK - 1) / WF_BLOCK, WF_BLOCK, smem, st>>>(sc, Lv, P, pixels,
+                                                                                        plan.classify ? 1 : 0, M);
+    else
+      k_wf_primary_trace<false><<<(pixels + WF_BLOCK - 1) / WF_BLOCK, WF_BLOCK, smem, st>>>(sc, Lv, P, pixels,
+                                                                                         plan.classify ? 1 : 0, M);
     mark(1, st);
   };
   // primary hits once per pixel per launch; kept behind the batch workspaces
@@ -746,6 +780,11 @@ int lt_launch_render_wavefront(const LtSceneDev& sc, const LtPlan& plan, const L
   if (plan.sharedPrimary && !views) {
     P = records(0, 0);
     trace_primary(L, P, stream);
+    preLaunches = 1;
+  } else if (list) {  // camera rays traced by k_wf_primary: only the film table, for the shade kernels
+    P = records(0, 0);
+    P.hits = nullptr;
+    k_wf_list_film<<<(pixels + WF_BLOCK - 1) / WF_BLOCK, WF_BLOCK, 0, stream>>>(L, P.film, M);
     preLaunches = 1;
   }
   if (overlap) {
@@ -796,19 +835,24 @@ int lt_launch_render_wavefront(const LtSceneDev& sc, const LtPlan& plan, const L
           if (g > smCount * 32) g = smCount * 32;
           mark(0, st, plan.sharedPrimary ? LT_TIMED_PRIMARY_SHADE : LT_TIMED_TRAVERSAL);
           if (stats)
-            k_wf_primary<true, true><<<g, WF_BLOCK, smem, st>>>(sc, Ls, B, segs[k].count, pixels, s, dCounters,
-                                                                segP[k], out, segs[k].at * pixels);
+            k_wf_primary<true, true, false><<<g, WF_BLOCK, smem, st>>>(sc, Ls, B, segs[k].count, pixels, s, dCounters,
+                                                                       segP[k], out, segs[k].at * pixels, M);
           else
-            k_wf_primary<false, true><<<g, WF_BLOCK, smem, st>>>(sc, Ls, B, segs[k].count, pixels, s, nullptr,
-                                                                 segP[k], out, segs[k].at * pixels);
+            k_wf_primary<false, true, false><<<g, WF_BLOCK, smem, st>>>(sc, Ls, B, segs[k].count, pixels, s, nullptr,
+                                                                        segP[k], out, segs[k].at * pixels, M);
           mark(1, st, plan.sharedPrimary ? LT_TIMED_PRIMARY_SHADE : LT_TIMED_TRAVERSAL);
         }
         launches += 1 + nSeg;
       } else {
         // a traversal kernel only when it traces the camera rays itself
         mark(0, st, plan.sharedPrimary ? LT_TIMED_PRIMARY_SHADE : LT_TIMED_TRAVERSAL);
-        if (stats) k_wf_primary<true, false><<<grid, WF_BLOCK, smem, st>>>(sc, Lb, B, nf, pixels, s, dCounters, P, out, 0);
-        else k_wf_primary<false, false><<<grid, WF_BLOCK, smem, st>>>(sc, Lb, B, nf, pixels, s, nullptr, P, out, 0);
+        if (list) {
+          if (stats) k_wf_primary<true, false, true><<<grid, WF_BLOCK, smem, st>>>(sc, Lb, B, nf, pixels, s, dCounters, P, out, 0, M);
+          else k_wf_primary<false, false, true><<<grid, WF_BLOCK, smem, st>>>(sc, Lb, B, nf, pixels, s, nullptr, P, out, 0, M);
+        } else {
+          if (stats) k_wf_primary<true, false, false><<<grid, WF_BLOCK, smem, st>>>(sc, Lb, B, nf, pixels, s, dCounters, P, out, 0, M);
+          else k_wf_primary<false, false, false><<<grid, WF_BLOCK, smem, st>>>(sc, Lb, B, nf, pixels, s, nullptr, P, out, 0, M);
+        }
         mark(1, st, plan.sharedPrimary ? LT_TIMED_PRIMARY_SHADE : LT_TIMED_TRAVERSAL);
         launches += 2;
       }
@@ -842,12 +886,15 @@ int lt_launch_render_wavefront(const LtSceneDev& sc, const LtPlan& plan, const L
       for (int k = 0; k < nSeg; k++) {
         LtWfBuffers Bs = B;
         Bs.frameCol = B.frameCol + (size_t)segs[k].at * pixels;
-        k_wf_accumulate<<<(pixels + WF_BLOCK - 1) / WF_BLOCK, WF_BLOCK, 0, st>>>(
-            segL[k], Bs, dOut + (size_t)segs[k].view * imageFloats, pixels, segs[k].first, segs[k].count, segP[k].cls);
+        k_wf_accumulate<false, false><<<(pixels + WF_BLOCK - 1) / WF_BLOCK, WF_BLOCK, 0, st>>>(
+            segL[k], Bs, dOut + (size_t)segs[k].view * imageFloats, pixels, segs[k].first, segs[k].count, segP[k].cls, M);
       }
       launches += nSeg;
     } else {
-      k_wf_accumulate<<<(pixels + WF_BLOCK - 1) / WF_BLOCK, WF_BLOCK, 0, st>>>(L, B, dOut, pixels, (int)pair0, nf, P.cls);
+      const int g = (pixels + WF_BLOCK - 1) / WF_BLOCK;
+      if (!list) k_wf_accumulate<false, false><<<g, WF_BLOCK, 0, st>>>(L, B, dOut, pixels, (int)pair0, nf, P.cls, M);
+      else if (!M.m2) k_wf_accumulate<true, false><<<g, WF_BLOCK, 0, st>>>(L, B, dOut, pixels, (int)pair0, nf, P.cls, M);
+      else k_wf_accumulate<true, true><<<g, WF_BLOCK, 0, st>>>(L, B, dOut, pixels, (int)pair0, nf, P.cls, M);
       launches++;
     }
     mark(1, st, LT_TIMED_ACCUMULATE);
