@@ -146,6 +146,14 @@ struct RenderExtensionB200 {
   Camera* const* ppViewCameras;   // viewCount cameras; pOutputBuffer holds viewCount images, view v at v * w * h * d
                                   // floats, each accumulated from zero within the call (lt_render_views); deviceCount
                                   // above 1 deals the views to the devices; built-in kernels only
+  // --- adaptive sampling (appended: older initialisers leave adaptiveError 0 = off) ---
+  float adaptiveError;            // > 0: render to this relative standard error per pixel (lt_render_adaptive): `frames`
+                                  // on every pixel, then rounds of adaptiveRoundFrames on the pixels still above it;
+                                  // needs accumulate; built-in kernels, one view, no sample split
+  uint32_t adaptiveRoundFrames;   // frames per later round (0 -> frames)
+  uint32_t adaptiveMaxFrames;     // most frames of a pixel (0 -> frames + 3 x round frames)
+  uint32_t* pPixelFrames;         // out (may be NULL): width * height frame counts, the frames each pixel received
+  uint32_t adaptiveRounds;        // out: rounds rendered
 };
 
 // ================================================================================================
@@ -518,7 +526,8 @@ public:
 // scene_parser.h -- JSON .scene file -> Camera / Model / AccelerationStructureExplicit / RenderProperties*
 // (reference: include/lens_trace/scene_parser.h, src/scene_parser.cpp; same keys, same defaults).
 // The JSON reader is this project's own (lens_trace_b200/host/scene_parser.cpp).  B200 additions,
-// all optional, under "renderer": "frames", "accumulate", "max_ray_depth", "devices", "split".
+// all optional, under "renderer": "frames", "accumulate", "max_ray_depth", "devices", "split", "adaptive_error",
+// "adaptive_round_frames", "adaptive_max_frames".
 // ================================================================================================
 struct RendererParsed {
   RenderPlatform renderPlatform = RENDER_PLATFORM_OPENCL;
@@ -535,6 +544,9 @@ struct RendererParsed {
   uint32_t maxRayDepth = 0;   // B200 (0 -> 16)
   uint32_t deviceCount = 0;   // B200: "devices" (GPUs 0..n-1 render each call together)
   uint32_t splitMode = 0;     // B200: "split": "samples" | "tiles" (default: chosen per call)
+  float adaptiveError = 0;          // B200: "adaptive_error" (> 0: adaptive sampling, RenderExtensionB200)
+  uint32_t adaptiveRoundFrames = 0; // B200: "adaptive_round_frames"
+  uint32_t adaptiveMaxFrames = 0;   // B200: "adaptive_max_frames"
 };
 
 struct CameraParsed {

@@ -58,6 +58,9 @@ uint64_t lth_write_synthetic_scene(const char* obj_path, uint32_t grid_n, uint64
 /* runs a .scene file end to end (SceneParser -> Renderer -> out); returns 0 on success */
 int lth_run_scene_file(const char* scene_path, float* out, uint64_t out_bytes, uint64_t dims_out[3]);
 
+/* the RenderExtensionB200 a .scene file gives the renderer, copied to ext_out (no device needed); 0 on success */
+int lth_scene_extension(const char* scene_path, void* ext_out);
+
 #ifdef __cplusplus
 }
 #endif

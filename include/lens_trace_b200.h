@@ -246,13 +246,82 @@ int lt_render_views_device(lt_ctx* ctx, lt_scene* scene, const void* cameras28, 
  * asynchronous on the context stream unless sync != 0.  An empty mask launches nothing more and returns LT_OK.
  * lt_last_stats describes the call as for lt_render_device; kernel_launches counts the compaction.
  * Not provided: a host-memory form or the context accumulator, multi-GPU contexts, views, plug-ins, the C++ renderer
- * (RenderExtensionB200), and any policy that chooses the mask: the caller decides which pixels need more frames. */
+ * (RenderExtensionB200), and any policy that chooses the mask: the caller decides which pixels need more frames.
+ * lt_render_adaptive (below) is one such policy inside the library, with a host form, multi-GPU contexts and the C++
+ * renderer. */
 int lt_render_masked_device(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params,
                             const uint8_t* device_mask, float* device_out, float* device_m2, int sync);
 /* Test hook (single-GPU contexts): reversed != 0 makes later lt_render_masked_device calls on ctx render their pixel
- * list in reverse order (one more kernel), 0 restores the compaction's order.  The output is the same either way; tests
+ * list, and lt_render_adaptive calls every list they render, in reverse order (one more kernel per list), 0 restores the
+ * compaction's order.  The output is the same either way; tests
  * compare the two. */
 int lt_debug_ctx_list_order(lt_ctx* ctx, int reversed);
+
+/* Adaptive sampling inside the library: render to a noise target.  The stopping rule is the relative standard error of
+ * each pixel's running mean (INTEGRATION.md section 5e); lt_render_masked_device stays the way to use a rule of one's
+ * own. */
+typedef struct lt_adaptive_params {
+  uint32_t struct_size;  /* = sizeof(lt_adaptive_params) */
+  float target;          /* a pixel stops once its relative standard error is <= target; finite, > 0 */
+  float floor;           /* the error is relative to max(mean, floor); 0 -> 1e-4; finite, >= 0 */
+  int32_t round_frames;  /* frames per round after the first; 0 -> params->frames; >= 0 */
+  int32_t max_frames;    /* most frames one pixel gets in this call; >= params->frames */
+} lt_adaptive_params;
+
+typedef struct lt_adaptive_result {
+  int32_t rounds;              /* rounds rendered, the first included (the maximum over devices) */
+  uint64_t pixel_frames;       /* sum over pixels of the frames this call rendered */
+  uint64_t pixels_unconverged; /* pixels that reached max_frames still above target */
+} lt_adaptive_result;
+
+/* Render every pixel, then keep rendering only the pixels whose relative standard error is above a target.
+ * Round schedule: round 1 renders every pixel for F1 = params->frames frames; round r + 1 renders
+ * min(round_frames, max_frames - (F1 + ... + Fr)) frames for the pixels that go on; the call stops when a round's list is
+ * empty or max_frames is reached.  Every pixel of a round has the same frames behind it, camera.frameCount + F1 + ... +
+ * Fr, so each round is a masked continuation (lt_render_masked_device) with m2.
+ * Stopping rule, after a round, in FP32 with one IEEE round-to-nearest per operation: n = camera.frameCount + F1 + ... +
+ * Fr, d = (float)n * (float)(n - 1), and per channel k < 3 e_k = sqrt(m2_k / d) / (mean_k < floor ? floor : mean_k).
+ * A pixel goes on to the next round if it was in this round, no e_k is NaN and some e_k > target (what torch's sqrt, /,
+ * clamp_min and amax(...) > target compute, NaN included).
+ * Result: every pixel p with frame count n_p holds bit for bit the mean lt_render_device gives with frames = n_p -
+ * camera.frameCount from the same starting contents, and the m2 lt_render_masked_device keeps; it depends neither on
+ * the order of the pixel lists nor on the device count.
+ * Checked before anything is launched (LT_ERR_INVALID): the parameters as lt_render; accum_mode other than
+ * LT_ACCUM_RUNNING_MEAN; frame_stride > 1; camera.frameCount + frames < 2; target not finite or <= 0, floor not finite
+ * or < 0, round_frames < 0, max_frames < frames.  An image of more than 2^31 - 1 pixels is LT_ERR_UNSUPPORTED.  Every
+ * kernel id is accepted; the deterministic ones have m2 = 0 and stop after round 1.  With LT_FLAG_STATS (single-GPU)
+ * the counters and kernel_launches are summed over the rounds; kernel_launches counts the list and selection kernels
+ * too, kernel_ms sums the rounds' render kernels.
+ * After each round a selection kernel writes the pixels that go on into the next list, and the call reads the list's
+ * length back (one 4-byte copy and a synchronisation of the context stream per round, no others).
+ * Host form: accumulates from zero (as lt_accum_reset + lt_render, per pixel) in buffers the context owns (grow-only:
+ * mean, m2, frame counts); neither reads nor changes the context accumulator.  host_out receives width * height * depth
+ * floats of means, host_frames (may be NULL) width * height frame counts n_p.  Synchronous.  On a multi-GPU context
+ * device g owns every G-th block of 8 image rows (as LT_SPLIT_TILES) and runs the whole loop on its rows on its own (no
+ * collective); split_mode must be LT_SPLIT_AUTO or LT_SPLIT_TILES (LT_ERR_INVALID otherwise), LT_FLAG_STATS is
+ * LT_ERR_UNSUPPORTED there as for lt_render.  out_result (may be NULL) receives the result. */
+int lt_render_adaptive(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params,
+                       const lt_adaptive_params* aparams, float* host_out, uint32_t* host_frames,
+                       lt_adaptive_result* out_result);
+/* The same in device memory of ctx's device (single-GPU contexts only, LT_ERR_UNSUPPORTED otherwise): device_out (width
+ * * height * depth floats) and device_m2 (required, width * height * 3 floats, 4-byte aligned) are the running mean and
+ * its Welford sums, continued from their contents: with camera.frameCount = c > 0 they must hold c frames for every
+ * pixel.  device_frames (may be NULL, 4-byte aligned) receives n_p for every pixel.  Memory of another device or of the
+ * host: LT_ERR_INVALID.  The count of the round that reaches max_frames is read back only when out_result is given;
+ * work after the last readback is asynchronous on the context stream unless sync != 0. */
+int lt_render_adaptive_device(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params,
+                              const lt_adaptive_params* aparams, float* device_out, float* device_m2,
+                              uint32_t* device_frames, lt_adaptive_result* out_result, int sync);
+/* Host-only (no device needed): the argument checks of lt_render_adaptive with the same codes and messages, then the
+ * frames of each round the call would render if every pixel kept going (F1, F2, ...), camera.frameCount being
+ * first_frame_count.  Returns the number of rounds (out_frames may be NULL to ask for it; LT_ERR_INVALID when capacity
+ * is too small), negative on error. */
+int lt_debug_adaptive_rounds(const lt_render_params* params, const lt_adaptive_params* aparams,
+                             uint32_t first_frame_count, int32_t* out_frames, int capacity);
+/* Test hook (single-GPU contexts): later adaptive calls on ctx render only the rows device `part` of a `parts`-device
+ * context would own (every parts-th block of 8 rows from block `part`) and leave the other pixels untouched, so that the
+ * multi-GPU partition can be tested on one GPU.  parts = 1, part = 0 restores the whole image. */
+int lt_debug_ctx_adaptive_part(lt_ctx* ctx, int parts, int part);
 
 /* The output buffer of the reference API is the caller's malloc'ed memory (pOutputBuffer, structures.h:62,76).
  * lt_render copies into such pageable memory through its own pinned staging buffer; an application that reuses one

@@ -22,7 +22,8 @@ SYMBOLS = [
     "lt_debug_plan", "lt_debug_ctx_limits", "lt_render_plugin_frames", "lt_debug_build_traversal_tree",
     "lt_debug_scene_traversal_tree", "lt_debug_traversal_tree", "lt_render_views", "lt_render_views_device",
     "lt_debug_plan_views", "lt_scene_refit", "lt_scene_refit_device", "lt_debug_scene_bytes",
-    "lt_render_masked_device", "lt_debug_plan_masked", "lt_debug_ctx_list_order",
+    "lt_render_masked_device", "lt_debug_plan_masked", "lt_debug_ctx_list_order", "lt_render_adaptive",
+    "lt_render_adaptive_device", "lt_debug_adaptive_rounds", "lt_debug_ctx_adaptive_part",
 ]
 
 
@@ -46,6 +47,22 @@ class Stats(C.Structure):
         ("trace_launches", C.c_int32), ("shade_ms", C.c_float), ("primary_shade_ms", C.c_float),
         ("accumulate_ms", C.c_float), ("shade_launches", C.c_int32),
     ]
+
+
+class AdaptiveParams(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("target", C.c_float), ("floor", C.c_float), ("round_frames", C.c_int32),
+                ("max_frames", C.c_int32)]
+
+
+class AdaptiveResult(C.Structure):
+    _fields_ = [("rounds", C.c_int32), ("pixel_frames", C.c_uint64), ("pixels_unconverged", C.c_uint64)]
+
+
+def make_adaptive(target, max_frames, round_frames=0, floor=0.0):
+    a = AdaptiveParams()
+    a.struct_size = C.sizeof(AdaptiveParams)
+    a.target, a.floor, a.round_frames, a.max_frames = target, floor, round_frames, max_frames
+    return a
 
 
 _lib = None
@@ -89,6 +106,14 @@ def load():
     lib.lt_render_masked_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(RenderParams), C.c_void_p,
                                             C.c_void_p, C.c_void_p, C.c_int]
     lib.lt_debug_ctx_list_order.argtypes = [C.c_void_p, C.c_int]
+    lib.lt_render_adaptive.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(RenderParams),
+                                       C.POINTER(AdaptiveParams), C.c_void_p, C.c_void_p, C.POINTER(AdaptiveResult)]
+    lib.lt_render_adaptive_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(RenderParams),
+                                              C.POINTER(AdaptiveParams), C.c_void_p, C.c_void_p, C.c_void_p,
+                                              C.POINTER(AdaptiveResult), C.c_int]
+    lib.lt_debug_adaptive_rounds.argtypes = [C.POINTER(RenderParams), C.POINTER(AdaptiveParams), C.c_uint32, C.c_void_p,
+                                             C.c_int]
+    lib.lt_debug_ctx_adaptive_part.argtypes = [C.c_void_p, C.c_int, C.c_int]
     lib.lt_accum_reset.argtypes = [C.c_void_p]
     lib.lt_accum_read.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64]
     lib.lt_primary_hits.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p,
@@ -303,6 +328,42 @@ class Context:
                                                      C.c_void_p(m2_ptr) if m2_ptr else None, 1 if sync else 0),
                     "lt_render_masked_device")
 
+    def render_adaptive(self, scene, camera, params, target, round_frames=0, max_frames=None, floor=0.0):
+        """lt_render_adaptive: params.frames frames on every pixel, then rounds of round_frames (0: params.frames) on
+        the pixels whose relative standard error is still above target, up to max_frames (None: params.frames + 3
+        rounds).  Returns (mean float32 [H, W, depth], frame counts uint32 [H, W], AdaptiveResult)."""
+        if max_frames is None:
+            max_frames = params.frames + 3 * (round_frames or params.frames)
+        a = make_adaptive(target, max_frames, round_frames, floor)
+        out = np.empty((params.height, params.width, params.depth), dtype=np.float32)
+        frames = np.empty((params.height, params.width), dtype=np.uint32)
+        res = AdaptiveResult()
+        cam = np.ascontiguousarray(camera, dtype=L.CAMERA)
+        self._check(self.lib.lt_render_adaptive(self.h, scene.h, cam.ctypes.data, C.byref(params), C.byref(a),
+                                                out.ctypes.data, frames.ctypes.data, C.byref(res)), "lt_render_adaptive")
+        return out, frames, res
+
+    def render_adaptive_device(self, scene, camera, params, out_ptr, m2_ptr, frames_ptr=None, target=0.05,
+                               round_frames=0, max_frames=None, floor=0.0, sync=False):
+        """lt_render_adaptive_device: the adaptive loop continued in device memory -- out_ptr (H * W * depth floats of
+        running mean), m2_ptr (H * W * 3 floats of Welford sums) and frames_ptr (H * W uint32, or None), e.g. torch CUDA
+        tensors' data_ptr().  Returns the AdaptiveResult."""
+        if max_frames is None:
+            max_frames = params.frames + 3 * (round_frames or params.frames)
+        a = make_adaptive(target, max_frames, round_frames, floor)
+        res = AdaptiveResult()
+        cam = np.ascontiguousarray(camera, dtype=L.CAMERA)
+        self._check(self.lib.lt_render_adaptive_device(self.h, scene.h, cam.ctypes.data, C.byref(params), C.byref(a),
+                                                       C.c_void_p(out_ptr), C.c_void_p(m2_ptr),
+                                                       C.c_void_p(frames_ptr) if frames_ptr else None, C.byref(res),
+                                                       1 if sync else 0), "lt_render_adaptive_device")
+        return res
+
+    def debug_adaptive_part(self, parts, part):
+        """Test hook: later adaptive calls render only the rows part `part` of a `parts`-device context would own
+        (parts=1, part=0: the whole image again)"""
+        self._check(self.lib.lt_debug_ctx_adaptive_part(self.h, parts, part), "lt_debug_ctx_adaptive_part")
+
     def accum_reset(self):
         self._check(self.lib.lt_accum_reset(self.h), "lt_accum_reset")
 
@@ -424,6 +485,21 @@ def tile_rows(height, devices, device):
     out = np.zeros(n, np.int32)
     lib.lt_debug_tile_rows(height, devices, device, out.ctypes.data, n)
     return out
+
+
+def adaptive_rounds(params, aparams, first_frame_count=0):
+    """Host-only: the frames of every round an adaptive call would render if every pixel kept going
+    (lt_debug_adaptive_rounds), after the call's argument checks; raises LtError with the call's code and message."""
+    lib = load()
+    n = lib.lt_debug_adaptive_rounds(C.byref(params), C.byref(aparams) if aparams is not None else None,
+                                     first_frame_count, None, 0)
+    if n < 0:
+        e = LtError("lt_render_adaptive failed (%d): %s" % (n, lib.lt_last_error(None).decode()))
+        e.code = n
+        raise e
+    out = np.zeros(n, np.int32)
+    lib.lt_debug_adaptive_rounds(C.byref(params), C.byref(aparams), first_frame_count, out.ctypes.data, n)
+    return [int(x) for x in out]
 
 
 PLAN_FIELDS = ("pipeline", "tree", "stats", "cull", "batch_frames", "streams", "rounds", "samples_per_frame",

@@ -215,6 +215,7 @@ extern "C" void lt_ctx_destroy(lt_ctx* ctx) {
   if (ctx->dViews) cudaFree(ctx->dViews);
   if (ctx->dViewFrameCounts) cudaFree(ctx->dViewFrameCounts);
   if (ctx->dMaskList) cudaFree(ctx->dMaskList);
+  if (ctx->dAdaptive) cudaFree(ctx->dAdaptive);
   delete ctx->copyPool;
   if (ctx->stage) cudaFreeHost(ctx->stage);
   for (cudaEvent_t e : ctx->stageEvents) cudaEventDestroy(e);
@@ -823,8 +824,28 @@ extern "C" int lt_render_device(lt_ctx* ctx, lt_scene* scene, const void* camera
   return render_common(ctx, scene, L, device_out, sync != 0);
 }
 
-// lt_render_masked_device: the pixel list in ctx->dMaskList, its count first, the list from kMaskListAt on (256 B)
-static const size_t kMaskListAt = 64;
+// lt_render_masked_device: the pixel list in ctx->dMaskList, its count first, the list from kMaskListAt on (256 B).
+// lt_render_adaptive: two lists (ping-pong between rounds), their counts at [0] and [1], the second list kListPad-aligned
+static const size_t kMaskListAt = 64, kListPad = 64;
+
+// The rendering of a masked call and of each adaptive round, given a ready list of `count` pixels in device memory: the
+// test hook's reversal, then the plan and the launches for the listed pixels.  An empty list launches nothing.
+static int render_listed(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, int* dList, int count, float* dOut,
+                         float* dM2, bool sync) {
+  if (count == 0) {  // nothing to render: no pixel is written
+    const int sms = ctx->stats.sm_count;
+    const float uploadMs = ctx->stats.upload_ms;
+    ctx->stats = lt_stats{};
+    ctx->stats.sm_count = sms;
+    ctx->stats.upload_ms = uploadMs;
+    return LT_OK;
+  }
+  const int extra = ctx->reverseList ? lt_launch_list_reverse(dList, count, ctx->stream) : 0;
+  const LtList list = {dList, count, dM2};
+  const int rc = render_common(ctx, scene, L, dOut, sync, nullptr, 1, &list);
+  ctx->stats.kernel_launches += extra;
+  return rc;
+}
 
 extern "C" int lt_render_masked_device(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params,
                                        const uint8_t* device_mask, float* device_out, float* device_m2, int sync) {
@@ -854,20 +875,187 @@ extern "C" int lt_render_masked_device(lt_ctx* ctx, lt_scene* scene, const void*
     CK(cudaMemcpyAsync(&count, dCount, sizeof count, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
   }
-  if (count == 0) {  // nothing to render: no pixel is written
-    const int sms = ctx->stats.sm_count;
-    const float uploadMs = ctx->stats.upload_ms;
-    ctx->stats = lt_stats{};
-    ctx->stats.sm_count = sms;
-    ctx->stats.upload_ms = uploadMs;
-    ctx->stats.kernel_launches = 1;
+  const int rc = render_listed(ctx, scene, L, dList, count, device_out, device_m2, sync != 0);
+  ctx->stats.kernel_launches += 1;  // the compaction
+  return rc;
+}
+
+// The adaptive loop on one device (arguments checked): round 1 over every pixel of the context's part of the image, then
+// rounds over the pixels the selection kernel keeps, each continuing from the frames all its pixels hold.  dOut, dM2 and
+// dFrames are full-size images.  One readback and stream synchronisation per round: the survivors' count, which the
+// next round's plan needs; the count of the round that reaches max_frames is read only when readLast.
+static int adaptive_loop(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, const LtAdaptive& A, float* dOut, float* dM2,
+                         unsigned* dFrames, int parts, int part, bool readLast, bool sync, lt_adaptive_result* res) {
+  CK(cudaSetDevice(ctx->device));
+  *res = lt_adaptive_result{};
+  const size_t pixels = (size_t)L.width * L.height, second = kMaskListAt + (pixels + kListPad - 1) / kListPad * kListPad;
+  CK(ctx_grow(&ctx->dMaskList, &ctx->maskListSize, second + pixels, sizeof(int)));
+  int* counts = ctx->dMaskList;
+  int* lists[2] = {ctx->dMaskList + kMaskListAt, ctx->dMaskList + second};
+  cudaStream_t st = ctx->stream;
+  // round 1: a full image is the NULL-mask list of lt_render_masked_device, so it plans as the unmasked call
+  int count = (int)pixels;
+  if (parts <= 1) {
+    lt_launch_mask_compact(nullptr, L.width, L.height, lists[0], &counts[0], st);
+  } else {
+    lt_launch_rows_compact(L.width, L.height, parts, part, lists[0], &counts[0], st);
+    count = lt_tile_rows_of(L.height, parts, part) * L.width;
+  }
+  CK(cudaGetLastError());
+  lt_stats sum = {};
+  sum.kernel_launches = 1;
+  int cur = 0, frames = L.frames, done = 0;
+  bool waited = true;  // the device has finished every round counted in sum.kernel_ms
+  while (count > 0) {
+    LtLaunch Lr = L;
+    Lr.frames = frames;
+    Lr.cam.frameCount = L.cam.frameCount + (unsigned)done;
+    if (int rc = render_listed(ctx, scene, Lr, lists[cur], count, dOut, dM2, false)) return rc;
+    const lt_stats& r = ctx->stats;
+    sum.rays += r.rays;
+    sum.node_tests += r.node_tests;
+    sum.tri_tests += r.tri_tests;
+    sum.kernel_launches += r.kernel_launches;
+    sum.trace_ms += r.trace_ms;
+    sum.trace_launches += r.trace_launches;
+    sum.shade_ms += r.shade_ms;
+    sum.primary_shade_ms += r.primary_shade_ms;
+    sum.accumulate_ms += r.accumulate_ms;
+    sum.shade_launches += r.shade_launches;
+    res->rounds++;
+    res->pixel_frames += (uint64_t)count * (uint64_t)frames;
+    done += frames;
+    const int nextFrames = lt_adaptive_next_frames(A, done);
+    const bool last = nextFrames == 0;
+    int* next = last ? nullptr : lists[1 - cur];
+    sum.kernel_launches += lt_launch_adaptive_select(lists[cur], count, dOut, L.depth, dM2, dFrames,
+                                                     L.cam.frameCount + (unsigned)done, A.target, A.floor, next,
+                                                     &counts[1 - cur], st);
+    CK(cudaGetLastError());
+    if (last && !readLast) {
+      waited = false;
+      break;
+    }
+    int kept = 0;
+    CK(cudaMemcpyAsync(&kept, &counts[1 - cur], sizeof kept, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    float ms = 0.0f;
+    CK(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+    sum.kernel_ms += ms;
+    if (last) {
+      res->pixels_unconverged = (uint64_t)kept;
+      break;
+    }
+    count = kept;
+    cur = 1 - cur;
+    frames = nextFrames;
+  }
+  if (!waited && sync) {
+    CK(cudaStreamSynchronize(st));
+    float ms = 0.0f;
+    CK(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+    sum.kernel_ms += ms;
+    waited = true;
+  }
+  sum.sm_count = ctx->stats.sm_count;
+  sum.upload_ms = ctx->stats.upload_ms;
+  if (!waited) sum.kernel_ms = 0.0f;  // not known before the work is done
+  ctx->stats = sum;
+  return LT_OK;
+}
+
+// the single-GPU checks of both adaptive forms (the multi-GPU form checks in lt_multi_render_adaptive)
+static int adaptive_args(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params,
+                         const lt_adaptive_params* aparams, const char* who, LtLaunch* L, LtAdaptive* A) {
+  if (!ctx) return fail(nullptr, LT_ERR_INVALID, std::string(who) + ": ctx is NULL");
+  if (!scene || !camera28 || !params) return fail(ctx, LT_ERR_INVALID, std::string(who) + ": NULL argument");
+  if (int rc = lt_params_to_launch(ctx, params, L, who)) return rc;
+  memcpy(&L->cam, camera28, sizeof(RefCamera));
+  return lt_adaptive_check(ctx, *L, aparams, who, A);
+}
+
+int lt_internal_render_adaptive(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, const LtAdaptive& A, float* host_out,
+                                uint32_t* host_frames, int parts, int part, lt_adaptive_result* res) {
+  CK(cudaSetDevice(ctx->device));
+  const size_t pixels = (size_t)L.width * L.height, meanFloats = pixels * L.depth;
+  CK(ctx_grow(&ctx->dAdaptive, &ctx->adaptiveFloats, meanFloats + 4 * pixels, sizeof(float)));
+  float* dMean = ctx->dAdaptive;
+  float* dM2 = dMean + meanFloats;
+  unsigned* dFrames = (unsigned*)(dM2 + 3 * pixels);
+  // from zero, as lt_accum_reset leaves the context accumulator
+  CK(cudaMemsetAsync(dMean, 0, (meanFloats + 3 * pixels) * sizeof(float), ctx->stream));
+  if (int rc = adaptive_loop(ctx, scene, L, A, dMean, dM2, host_frames ? dFrames : nullptr, parts, part, true, true, res))
+    return rc;
+  if (parts <= 1) {
+    if (host_out)
+      if (int rc = lt_internal_download(ctx, host_out, dMean, meanFloats * sizeof(float))) return rc;
+    if (host_frames)
+      if (int rc = lt_internal_download(ctx, (float*)host_frames, (const float*)dFrames, pixels * sizeof(unsigned)))
+        return rc;
     return LT_OK;
   }
-  const int extra = ctx->reverseList ? lt_launch_list_reverse(dList, count, ctx->stream) : 0;
-  const LtList list = {dList, count, device_m2};
-  const int rc = render_common(ctx, scene, L, device_out, sync != 0, nullptr, 1, &list);
-  ctx->stats.kernel_launches += 1 + extra;  // the compaction (and the test hook's reversal)
+  // a part's rows only: the blocks of the row partition, out of the full-size buffers
+  const int rows = lt_tile_rows_of(L.height, parts, part);
+  const size_t meanRow = (size_t)L.width * L.depth * sizeof(float), frameRow = (size_t)L.width * sizeof(unsigned);
+  const size_t blockRows = (size_t)parts * LT_TILE_ROWS, first = (size_t)part * LT_TILE_ROWS;
+  cudaError_t e = cudaSuccess;
+  if (host_out && rows > 0)
+    e = lt_copy_row_blocks(host_out, (const char*)dMean + first * meanRow, blockRows * meanRow, meanRow, rows, parts,
+                           part, ctx->stream);
+  if (e == cudaSuccess && host_frames && rows > 0)
+    e = lt_copy_row_blocks(host_frames, (const char*)dFrames + first * frameRow, blockRows * frameRow, frameRow, rows,
+                           parts, part, ctx->stream);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+  if (e != cudaSuccess) return fail(ctx, LT_ERR_CUDA, std::string("lt_render_adaptive: row copy: ") + cudaGetErrorString(e));
+  return LT_OK;
+}
+
+extern "C" int lt_render_adaptive(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params,
+                                  const lt_adaptive_params* aparams, float* host_out, uint32_t* host_frames,
+                                  lt_adaptive_result* out_result) {
+  if (ctx && ctx->group)
+    return lt_multi_render_adaptive(ctx, scene, camera28, params, aparams, host_out, host_frames, out_result);
+  LtLaunch L;
+  LtAdaptive A;
+  if (int rc = adaptive_args(ctx, scene, camera28, params, aparams, "lt_render_adaptive", &L, &A)) return rc;
+  lt_adaptive_result res;
+  const int rc =
+      lt_internal_render_adaptive(ctx, scene, L, A, host_out, host_frames, ctx->adaptiveParts, ctx->adaptivePart, &res);
+  if (rc == LT_OK && out_result) *out_result = res;
   return rc;
+}
+
+extern "C" int lt_render_adaptive_device(lt_ctx* ctx, lt_scene* scene, const void* camera28,
+                                         const lt_render_params* params, const lt_adaptive_params* aparams,
+                                         float* device_out, float* device_m2, uint32_t* device_frames,
+                                         lt_adaptive_result* out_result, int sync) {
+  const char* who = "lt_render_adaptive_device";
+  const std::string w = std::string(who) + ": ";
+  if (ctx && ctx->group)
+    return fail(ctx, LT_ERR_UNSUPPORTED, w + "a multi-GPU context renders into host memory (lt_render_adaptive)");
+  LtLaunch L;
+  LtAdaptive A;
+  if (int rc = adaptive_args(ctx, scene, camera28, params, aparams, who, &L, &A)) return rc;
+  if (!device_out || !device_m2) return fail(ctx, LT_ERR_INVALID, w + "device_out and device_m2 are required");
+  if (int rc = check_device_memory(ctx, device_out, alignof(float), w, "device_out")) return rc;
+  if (int rc = check_device_memory(ctx, device_m2, alignof(float), w, "device_m2")) return rc;
+  if (device_frames)
+    if (int rc = check_device_memory(ctx, device_frames, alignof(uint32_t), w, "device_frames")) return rc;
+  lt_adaptive_result res;
+  const int rc = adaptive_loop(ctx, scene, L, A, device_out, device_m2, device_frames, ctx->adaptiveParts,
+                               ctx->adaptivePart, out_result != nullptr, sync != 0, &res);
+  if (rc == LT_OK && out_result) *out_result = res;
+  return rc;
+}
+
+extern "C" int lt_debug_ctx_adaptive_part(lt_ctx* ctx, int parts, int part) {
+  if (!ctx) return fail(nullptr, LT_ERR_INVALID, "lt_debug_ctx_adaptive_part: ctx is NULL");
+  if (ctx->group) return fail(ctx, LT_ERR_UNSUPPORTED, "lt_debug_ctx_adaptive_part: not available on a multi-GPU context");
+  if (parts < 1 || part < 0 || part >= parts)
+    return fail(ctx, LT_ERR_INVALID, "lt_debug_ctx_adaptive_part: needs parts >= 1 and 0 <= part < parts");
+  ctx->adaptiveParts = parts;
+  ctx->adaptivePart = part;
+  return LT_OK;
 }
 
 extern "C" int lt_debug_ctx_list_order(lt_ctx* ctx, int reversed) {

@@ -16,6 +16,11 @@
 struct lt_ctx;
 int lt_internal_ctx_device(const lt_ctx* ctx);  // lt_capi.cu
 
+// A row partition of an image into parts: part g owns every parts-th block of LT_TILE_ROWS rows from block g (the tile
+// split of a multi-GPU context, lt_render_adaptive's partition of its devices).  lt_tile_rows_of: the rows part g owns.
+#define LT_TILE_ROWS 8
+int lt_tile_rows_of(int height, int parts, int g);  // lt_multi.cu
+
 // ---- launch plan (lt_plan.cpp: lt_plan_render): every choice of which kernels run, on which tree, at which sizes ----
 // k_flat, k_flat_stream, k_path, or the wavefront pipeline (lt_wavefront.cu)
 enum LtPipeline { LT_PIPE_FLAT, LT_PIPE_FLAT_STREAM, LT_PIPE_PATH, LT_PIPE_WAVEFRONT };
@@ -61,6 +66,17 @@ int lt_params_normalise(lt_ctx* ctx, const lt_render_params* params, const std::
 int lt_params_to_launch(lt_ctx* ctx, const lt_render_params* params, LtLaunch* L, const char* who = "lt_render");
 // LT_ERR_UNSUPPORTED (message set) for an image a masked call cannot number with 32-bit pixel indices
 int lt_masked_image_check(lt_ctx* ctx, const LtLaunch& L, const char* who);
+// lt_render_adaptive's parameters after their checks: defaults applied (floor 0 -> 1e-4, round_frames 0 -> frames)
+struct LtAdaptive {
+  float target, floor;
+  int roundFrames, maxFrames;
+};
+// The checks of lt_render_adaptive that need no device, on the launch lt_params_to_launch made (camera included)
+int lt_adaptive_check(lt_ctx* ctx, const LtLaunch& L, const lt_adaptive_params* a, const char* who, LtAdaptive* out);
+// frames of the round that follows `done` frames of the call, 0 when max_frames is reached
+inline int lt_adaptive_next_frames(const LtAdaptive& A, int done) {
+  return A.maxFrames - done < A.roundFrames ? A.maxFrames - done : A.roundFrames;
+}
 
 // ---- host tree builders (lt_tree.cpp) ----
 // Host-side validation of the reference node array (bounds of every index the kernels will follow) and the depth the
@@ -86,6 +102,13 @@ int lt_launch_render(const LtSceneDev& sc, const LtPlan& plan, const LtLaunch& L
 int lt_launch_mask_compact(const unsigned char* dMask, int width, int height, int* dList, int* dCount,
                            cudaStream_t stream);
 int lt_launch_list_reverse(int* dList, int count, cudaStream_t stream);  // the list in reverse order, in place
+// lt_render_adaptive: the first list of part `part` of a `parts`-way row partition (k_rows_compact), and the selection
+// after a round of `count` listed pixels with n frames each: pixels that go on -> dNext (nullptr: only counted), their
+// number -> *dNextCount, n -> dFrames[pixel] when given (k_adaptive_select)
+int lt_launch_rows_compact(int width, int height, int parts, int part, int* dList, int* dCount, cudaStream_t stream);
+int lt_launch_adaptive_select(const int* dList, int count, const float* dMean, int depth, const float* dM2,
+                              unsigned* dFrames, unsigned n, float target, float floor, int* dNext, int* dNextCount,
+                              cudaStream_t stream);
 int lt_launch_primary_hits(const LtSceneDev& sc, const LtPlan& plan, const RefCamera& cam, int kernel, int flags,
                            int width, int height, int* dIds, int* dHit, float* dTuv, cudaStream_t stream);
 // Dynamic shared memory beyond 48 KB needs an opt-in per kernel and device: given once for every traversal kernel
@@ -200,6 +223,9 @@ struct lt_ctx {
   int* dMaskList = nullptr;  // lt_render_masked_device: the listed pixels' count, then (from kMaskListAt) the list
   size_t maskListSize = 0;
   bool reverseList = false;  // lt_debug_ctx_list_order: masked calls render their list in reverse order
+  float* dAdaptive = nullptr;  // host-form lt_render_adaptive: mean, m2 (3 per pixel), frame counts (one per pixel)
+  size_t adaptiveFloats = 0;
+  int adaptiveParts = 1, adaptivePart = 0;  // lt_debug_ctx_adaptive_part: adaptive calls render this part's rows only
   size_t totalMem = 0;
   char* stage = nullptr;  // pinned staging buffer of lt_render's copy into a pageable destination
   size_t stageBytes = 0;
@@ -258,6 +284,17 @@ int lt_internal_render_views(lt_ctx* ctx, lt_scene* scene, const RefCamera* cams
                              const lt_render_params* params, float* host_out, int hostFirst, int hostStride);
 int lt_multi_render_views(lt_ctx* ctx, lt_scene* scene, const RefCamera* cams, int count, const lt_render_params* params,
                           float* host_out);
+// lt_render_adaptive's host form on one device (arguments checked; L.cam is the camera): the rows of part `part` of a
+// `parts`-way row partition, from zero in the context's buffers, copied to their places in host_out / host_frames
+int lt_internal_render_adaptive(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, const LtAdaptive& A, float* host_out,
+                                uint32_t* host_frames, int parts, int part, lt_adaptive_result* res);
+int lt_multi_render_adaptive(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params,
+                             const lt_adaptive_params* aparams, float* host_out, uint32_t* host_frames,
+                             lt_adaptive_result* out_result);
+// Row blocks k, k + G, ... of a row partition (`rows` rows) from device memory, srcPitch bytes per block apart from src,
+// to their places in the host image dst (rowBytes per image row); asynchronous on `stream`
+cudaError_t lt_copy_row_blocks(void* dst, const void* src, size_t srcPitch, size_t rowBytes, int rows, int G, int k,
+                               cudaStream_t stream);
 // params->frames frames of a plug-in into ctx->dOut, combined by params->accum_mode (arguments already checked); `who`
 // names the entry point in error messages
 int lt_internal_render_plugin(lt_ctx* ctx, lt_scene* scene, const RefCamera& cam, const lt_render_params& P,

@@ -430,6 +430,57 @@ __global__ void k_list_reverse(int* __restrict__ list, int count) {
   list[count - 1 - i] = a;
 }
 
+// Appends the pixel of every lane with `set` to list at *count, in lane order, with one atomic per warp (the whole warp
+// calls it, as k_mask_compact appends); list == nullptr only counts.
+__device__ __forceinline__ void warp_append(bool set, int pixel, int* __restrict__ list, int* __restrict__ count) {
+  const unsigned lane = threadIdx.x & 31u, m = __ballot_sync(0xffffffffu, set);
+  if (m == 0u) return;
+  int base = 0;
+  if (lane == 0u) base = atomicAdd(count, __popc(m));
+  base = __shfl_sync(0xffffffffu, base, 0);
+  if (set && list) list[base + __popc(m & ((1u << lane) - 1u))] = pixel;
+}
+
+// The first list of an adaptive call on one part of a row partition (lt_render_adaptive on a multi-GPU context, and
+// lt_debug_ctx_adaptive_part): the pixels of every parts-th block of LT_TILE_ROWS rows from block `part`, in the order
+// k_mask_compact lists a full image.  The 16x8 tiles of thread_pixel lie inside one row block, so whole tiles are listed.
+__global__ void __launch_bounds__(LT_BLOCK) k_rows_compact(int width, int height, int parts, int part,
+                                                           int* __restrict__ list, int* __restrict__ count) {
+  int px, py;
+  const bool valid = thread_pixel(width, height, px, py);
+  warp_append(valid && (py / LT_TILE_ROWS) % parts == part, py * width + px, list, count);
+}
+
+// lt_render_adaptive's stopping rule after a round of `count` listed pixels, each with n frames behind it: thread i
+// looks at pixel list[i], records n in frames (when given), and the pixel goes on when no channel's relative standard
+// error e_k = sqrt(m2_k / (n (n - 1))) / max(mean_k, floor) is NaN and one exceeds target (FP32, one rounding per
+// operation; a NaN mean is kept by the comparison, as torch's clamp_min keeps it).  The pixels that go on are appended to
+// `next` as k_mask_compact appends, so a warp's run of a tile stays together and the next round's camera rays stay
+// coherent; next == nullptr (the round that reaches max_frames) only counts them.  Reads 28 B per listed pixel at depth 3.
+__global__ void __launch_bounds__(LT_BLOCK) k_adaptive_select(const int* __restrict__ list, int count,
+                                                              const float* __restrict__ mean, int depth,
+                                                              const float* __restrict__ m2, unsigned* __restrict__ frames,
+                                                              unsigned n, float target, float floor,
+                                                              int* __restrict__ next, int* __restrict__ nextCount) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  int pixel = 0;
+  bool more = false;
+  if (i < count) {
+    pixel = list[i];
+    if (frames) frames[pixel] = n;
+    const float d = __fmul_rn((float)n, (float)(n - 1u));
+    bool nan = false, above = false;
+    for (int k = 0; k < 3; k++) {
+      const float mk = mean[(long long)pixel * depth + k];
+      const float e = __fdiv_rn(__fsqrt_rn(__fdiv_rn(m2[3ll * pixel + k], d)), mk < floor ? floor : mk);
+      nan |= e != e;
+      above |= e > target;
+    }
+    more = !nan && above;
+  }
+  warp_append(more, pixel, next, nextCount);
+}
+
 // ------------------------------------------------------------------------------------------------
 // host-side launchers
 // ------------------------------------------------------------------------------------------------
@@ -443,6 +494,22 @@ int lt_launch_mask_compact(const unsigned char* dMask, int width, int height, in
                            cudaStream_t stream) {
   cudaMemsetAsync(dCount, 0, sizeof(int), stream);
   k_mask_compact<<<((width + 15) / 16) * ((height + 7) / 8), LT_BLOCK, 0, stream>>>(dMask, width, height, dList, dCount);
+  return 1;
+}
+
+int lt_launch_rows_compact(int width, int height, int parts, int part, int* dList, int* dCount, cudaStream_t stream) {
+  cudaMemsetAsync(dCount, 0, sizeof(int), stream);
+  k_rows_compact<<<((width + 15) / 16) * ((height + 7) / 8), LT_BLOCK, 0, stream>>>(width, height, parts, part, dList,
+                                                                                     dCount);
+  return 1;
+}
+
+int lt_launch_adaptive_select(const int* dList, int count, const float* dMean, int depth, const float* dM2,
+                              unsigned* dFrames, unsigned n, float target, float floor, int* dNext, int* dNextCount,
+                              cudaStream_t stream) {
+  cudaMemsetAsync(dNextCount, 0, sizeof(int), stream);
+  k_adaptive_select<<<(count + LT_BLOCK - 1) / LT_BLOCK, LT_BLOCK, 0, stream>>>(dList, count, dMean, depth, dM2, dFrames,
+                                                                                n, target, floor, dNext, dNextCount);
   return 1;
 }
 

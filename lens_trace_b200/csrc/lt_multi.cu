@@ -27,8 +27,6 @@
 
 #include "lt_internal.h"
 
-#define LT_TILE_ROWS 8
-
 namespace {
 
 struct NcclApi {
@@ -328,7 +326,7 @@ static bool ensure_peers(LtGroup* g, size_t floats, std::string* why) {
 }
 
 // rows of the image device g of G renders in a tile split: every G-th block of LT_TILE_ROWS rows
-static int tile_rows_of(int height, int G, int g) {
+int lt_tile_rows_of(int height, int G, int g) {
   int rows = 0;
   for (int b = g; b * LT_TILE_ROWS < height; b += G) {
     int left = height - b * LT_TILE_ROWS;
@@ -337,12 +335,31 @@ static int tile_rows_of(int height, int G, int g) {
   return rows;
 }
 
+// Row blocks k, k + G, ... of an image (`rows` rows in all, LT_TILE_ROWS per block, the last block shorter when the image
+// ends inside it) from device memory to their places in the host image dst: full blocks in one strided copy, a shorter
+// last block on its own.  The source holds the blocks srcPitch bytes apart from src (a device's own rows, or its blocks
+// inside a full-size image).  Asynchronous on `stream`.
+cudaError_t lt_copy_row_blocks(void* dst, const void* src, size_t srcPitch, size_t rowBytes, int rows, int G, int k,
+                               cudaStream_t stream) {
+  const int fullBlocks = rows / LT_TILE_ROWS, tail = rows % LT_TILE_ROWS;
+  const size_t dstPitch = (size_t)G * LT_TILE_ROWS * rowBytes;
+  char* d = (char*)dst + (size_t)k * LT_TILE_ROWS * rowBytes;
+  cudaError_t e = cudaSuccess;
+  if (fullBlocks > 0)
+    e = cudaMemcpy2DAsync(d, dstPitch, src, srcPitch, LT_TILE_ROWS * rowBytes, fullBlocks, cudaMemcpyDeviceToHost,
+                          stream);
+  if (e == cudaSuccess && tail > 0)
+    e = cudaMemcpyAsync(d + (size_t)fullBlocks * dstPitch, (const char*)src + (size_t)fullBlocks * srcPitch,
+                        tail * rowBytes, cudaMemcpyDeviceToHost, stream);
+  return e;
+}
+
 // Host-only (no device needed): the image rows device `device` of `devices` renders in a tile split, in the order of
 // its local rows -- the mapping the kernels apply (lt_device.cuh: lt_image_row) to the row count lt_multi_render hands
 // them.  Exposed so that the partition can be checked on a machine without a GPU.
 extern "C" int lt_debug_tile_rows(int height, int devices, int device, int32_t* out_rows, int capacity) {
   if (height < 1 || devices < 1 || device < 0 || device >= devices) return LT_ERR_INVALID;
-  const int rows = tile_rows_of(height, devices, device);
+  const int rows = lt_tile_rows_of(height, devices, device);
   if (out_rows) {
     if (capacity < rows) return LT_ERR_INVALID;
     for (int j = 0; j < rows; j++) {
@@ -393,7 +410,7 @@ int lt_multi_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt
 
   if (split == LT_SPLIT_TILES) {
     std::vector<int> rows(G);
-    for (int k = 0; k < G; k++) rows[k] = tile_rows_of(P.height, G, k);
+    for (int k = 0; k < G; k++) rows[k] = lt_tile_rows_of(P.height, G, k);
     const size_t rowBytes = (size_t)P.width * P.depth * sizeof(float);
     for (int k = 0; k < G; k++)
       workers.emplace_back([&, k]() {
@@ -407,17 +424,7 @@ int lt_multi_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt
         Pk.split_mode = 0;
         rcs[k] = lt_internal_render_rows(c, scene->parts[k], &cam, &Pk, c->dOut, P.height, LT_TILE_ROWS, G, k, 0);
         if (rcs[k] != LT_OK || !host_out) return;
-        // blocks k, k+G, ... of the image: full blocks in one strided copy, a shorter last block on its own
-        const int fullBlocks = rows[k] / LT_TILE_ROWS, tail = rows[k] % LT_TILE_ROWS;
-        char* dst = (char*)host_out + (size_t)k * LT_TILE_ROWS * rowBytes;
-        cudaError_t e = cudaSuccess;
-        if (fullBlocks > 0)
-          e = cudaMemcpy2DAsync(dst, (size_t)G * LT_TILE_ROWS * rowBytes, c->dOut, LT_TILE_ROWS * rowBytes,
-                                LT_TILE_ROWS * rowBytes, fullBlocks, cudaMemcpyDeviceToHost, c->stream);
-        if (e == cudaSuccess && tail > 0)
-          e = cudaMemcpyAsync(dst + (size_t)fullBlocks * G * LT_TILE_ROWS * rowBytes,
-                              (const char*)c->dOut + (size_t)fullBlocks * LT_TILE_ROWS * rowBytes, tail * rowBytes,
-                              cudaMemcpyDeviceToHost, c->stream);
+        cudaError_t e = lt_copy_row_blocks(host_out, c->dOut, LT_TILE_ROWS * rowBytes, rowBytes, rows[k], G, k, c->stream);
         if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
         if (e != cudaSuccess) rcs[k] = lt_internal_fail(c, LT_ERR_CUDA, std::string("tile copy: ") + cudaGetErrorString(e));
       });
@@ -569,6 +576,59 @@ int lt_multi_render_views(lt_ctx* ctx, lt_scene* scene, const RefCamera* cams, i
     if (c->stats.kernel_ms > ctx->stats.kernel_ms) ctx->stats.kernel_ms = c->stats.kernel_ms;
     ctx->stats.kernel_launches += c->stats.kernel_launches;
   }
+  cudaSetDevice(g->ctx[0]->device);
+  return LT_OK;
+}
+
+// lt_render_adaptive on several devices: device k runs the whole adaptive loop on its own rows of the row partition (every
+// G-th block of LT_TILE_ROWS rows from block k) in full-size buffers of its own context, and copies those rows of the
+// mean and the frame counts into the host buffers.  Every pixel's rounds depend on that pixel alone, so the result is
+// the single-GPU call's, and no collective is needed.
+int lt_multi_render_adaptive(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params,
+                             const lt_adaptive_params* aparams, float* host_out, uint32_t* host_frames,
+                             lt_adaptive_result* out_result) {
+  LtGroup* g = ctx->group;
+  const std::string who = "lt_render_adaptive: ";
+  if (!scene || !camera28 || !params) return lt_internal_fail(ctx, LT_ERR_INVALID, who + "NULL argument");
+  if (scene->parts.size() != g->ctx.size())
+    return lt_internal_fail(ctx, LT_ERR_INVALID, who + "the scene was not uploaded through this multi-GPU context");
+  lt_render_params P;
+  if (int rc = lt_params_normalise(ctx, params, who, &P)) return rc;
+  if (P.split_mode != LT_SPLIT_AUTO && P.split_mode != LT_SPLIT_TILES)
+    return lt_internal_fail(ctx, LT_ERR_INVALID, who + "the devices share the image by rows: split_mode must be LT_SPLIT_AUTO or LT_SPLIT_TILES");
+  P.split_mode = LT_SPLIT_AUTO;
+  // every check of the single-GPU call, before any device works
+  LtLaunch L;
+  if (int rc = lt_params_to_launch(ctx, &P, &L, "lt_render_adaptive")) return rc;
+  memcpy(&L.cam, camera28, sizeof(RefCamera));
+  LtAdaptive A;
+  if (int rc = lt_adaptive_check(ctx, L, aparams, "lt_render_adaptive", &A)) return rc;
+  if (P.flags & LT_FLAG_STATS)
+    return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED, who + "LT_FLAG_STATS counts on a single-GPU context");
+  const int G = (int)g->ctx.size();
+  std::vector<int> rcs(G, LT_OK);
+  std::vector<lt_adaptive_result> res(G, lt_adaptive_result{});
+  std::vector<std::thread> workers;
+  for (int k = 0; k < G; k++)
+    workers.emplace_back([&, k]() {
+      rcs[k] = lt_internal_render_adaptive(g->ctx[k], scene->parts[k], L, A, host_out, host_frames, G, k, &res[k]);
+    });
+  for (std::thread& t : workers) t.join();
+  for (int k = 0; k < G; k++)
+    if (rcs[k] != LT_OK) return lt_internal_fail(ctx, rcs[k], lt_last_error(g->ctx[k]));
+  lt_adaptive_result r = {};
+  ctx->stats.kernel_ms = 0.0f;
+  ctx->stats.kernel_launches = 0;
+  for (int k = 0; k < G; k++) {
+    if (res[k].rounds > r.rounds) r.rounds = res[k].rounds;
+    r.pixel_frames += res[k].pixel_frames;
+    r.pixels_unconverged += res[k].pixels_unconverged;
+    // statistics of the call: the slowest device's kernels, all devices' launches
+    const lt_ctx* c = g->ctx[k];
+    if (c->stats.kernel_ms > ctx->stats.kernel_ms) ctx->stats.kernel_ms = c->stats.kernel_ms;
+    ctx->stats.kernel_launches += c->stats.kernel_launches;
+  }
+  if (out_result) *out_result = r;
   cudaSetDevice(g->ctx[0]->device);
   return LT_OK;
 }

@@ -4,6 +4,7 @@
 #include "lens_trace_b200.h"
 #include "lt_internal.h"
 
+#include <float.h>
 #include <limits.h>
 #include <stddef.h>
 #include <string.h>
@@ -232,6 +233,54 @@ int lt_masked_image_check(lt_ctx* ctx, const LtLaunch& L, const char* who) {
     return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED,
                             std::string(who) + ": a masked call handles at most 2^31 - 1 pixels (width * height)");
   return LT_OK;
+}
+
+// lt_render_adaptive's own checks, after those of lt_render (L) and before anything is launched; then the image size
+int lt_adaptive_check(lt_ctx* ctx, const LtLaunch& L, const lt_adaptive_params* a, const char* who, LtAdaptive* out) {
+  const std::string w = std::string(who) + ": ";
+  if (!a) return lt_internal_fail(ctx, LT_ERR_INVALID, w + "aparams is NULL");
+  if (a->struct_size != sizeof(lt_adaptive_params))
+    return lt_internal_fail(ctx, LT_ERR_INVALID, w + "aparams.struct_size mismatch");
+  // the stopping rule reads the Welford sums, which only a running mean over consecutive frames keeps
+  if (L.accumMode != LT_ACCUM_RUNNING_MEAN || L.frameStride > 1)
+    return lt_internal_fail(ctx, LT_ERR_INVALID, w + "needs accum_mode LT_ACCUM_RUNNING_MEAN and frame_stride <= 1");
+  if ((long long)L.cam.frameCount + L.frames < 2)
+    return lt_internal_fail(ctx, LT_ERR_INVALID, w + "camera.frameCount + frames must be >= 2 (a variance needs two frames)");
+  if (!(a->target > 0.0f) || !(a->target <= FLT_MAX))
+    return lt_internal_fail(ctx, LT_ERR_INVALID, w + "target must be finite and > 0");
+  if (!(a->floor >= 0.0f) || !(a->floor <= FLT_MAX))
+    return lt_internal_fail(ctx, LT_ERR_INVALID, w + "floor must be finite and >= 0");
+  if (a->round_frames < 0) return lt_internal_fail(ctx, LT_ERR_INVALID, w + "round_frames must be >= 0");
+  if (a->max_frames < L.frames) return lt_internal_fail(ctx, LT_ERR_INVALID, w + "max_frames must be >= frames");
+  if ((long long)L.cam.frameCount + a->max_frames > (long long)UINT_MAX)
+    return lt_internal_fail(ctx, LT_ERR_INVALID, w + "camera.frameCount + max_frames must fit 32 bits");
+  if (int rc = lt_masked_image_check(ctx, L, who)) return rc;
+  out->target = a->target;
+  out->floor = a->floor == 0.0f ? 1e-4f : a->floor;
+  out->roundFrames = a->round_frames ? a->round_frames : L.frames;
+  out->maxFrames = a->max_frames;
+  return LT_OK;
+}
+
+extern "C" int lt_debug_adaptive_rounds(const lt_render_params* params, const lt_adaptive_params* aparams,
+                                        uint32_t first_frame_count, int32_t* out_frames, int capacity) {
+  const char* who = "lt_render_adaptive";
+  if (!params) return lt_internal_fail(nullptr, LT_ERR_INVALID, std::string(who) + ": NULL argument");
+  LtLaunch L = {};
+  if (int rc = lt_params_to_launch(nullptr, params, &L, who)) return rc;
+  L.cam.frameCount = first_frame_count;
+  LtAdaptive A;
+  if (int rc = lt_adaptive_check(nullptr, L, aparams, who, &A)) return rc;
+  int rounds = 0;
+  for (int done = 0, f = L.frames; f > 0; done += f, f = lt_adaptive_next_frames(A, done)) {
+    if (out_frames) {
+      if (rounds >= capacity)
+        return lt_internal_fail(nullptr, LT_ERR_INVALID, "lt_debug_adaptive_rounds: capacity is too small");
+      out_frames[rounds] = f;
+    }
+    rounds++;
+  }
+  return rounds;
 }
 
 static int debug_plan(const char* who, const lt_render_params* params, int views, uint64_t node_count,

@@ -21,6 +21,7 @@ SYMBOLS = [
     "lth_camera_create", "lth_camera_destroy", "lth_camera_buffer", "lth_camera_set_frame_count",
     "lth_camera_increment_frame_count", "lth_camera_set_position", "lth_camera_set_rotation", "lth_renderer_create",
     "lth_renderer_destroy", "lth_renderer_cached_scenes", "lth_render", "lth_write_synthetic_scene", "lth_run_scene_file", "lth_render_opencl",
+    "lth_scene_extension",
 ]
 
 
@@ -30,6 +31,8 @@ class RenderExtensionB200(C.Structure):
         ("maxRayDepth", C.c_uint32), ("collectStats", C.c_uint32), ("rays", C.c_uint64), ("nodeTests", C.c_uint64),
         ("triTests", C.c_uint64), ("kernelMilliseconds", C.c_float), ("deviceCount", C.c_uint32),
         ("splitMode", C.c_uint32), ("viewCount", C.c_uint32), ("ppViewCameras", C.c_void_p),
+        ("adaptiveError", C.c_float), ("adaptiveRoundFrames", C.c_uint32), ("adaptiveMaxFrames", C.c_uint32),
+        ("pPixelFrames", C.c_void_p), ("adaptiveRounds", C.c_uint32),
     ]
 
 
@@ -77,6 +80,7 @@ def load():
     lib.lth_render_opencl.restype = None
     lib.lth_write_synthetic_scene.argtypes = [C.c_char_p, C.c_uint32, u64]
     lib.lth_run_scene_file.argtypes = [C.c_char_p, vp, u64, C.POINTER(u64 * 3)]
+    lib.lth_scene_extension.argtypes = [C.c_char_p, vp]
     _lib = lib
     return lib
 
@@ -187,9 +191,13 @@ class Renderer:
 
 
 def make_extension(frames=1, accumulate=False, max_ray_depth=0, collect_stats=False, devices=0, split=0,
-                   view_cameras=None):
+                   view_cameras=None, adaptive_error=0.0, adaptive_round_frames=0, adaptive_max_frames=0,
+                   pixel_frames=None):
     """view_cameras: a list of Camera objects rendered in one call (viewCount, ppViewCameras) instead of the camera
-    given to render(); its `out` then holds len(view_cameras) images."""
+    given to render(); its `out` then holds len(view_cameras) images.
+    adaptive_error > 0: adaptive sampling to that relative standard error (lt_render_adaptive; needs accumulate);
+    pixel_frames: a C-contiguous uint32 array of H * W that receives each pixel's frame count; the rounds rendered
+    arrive in e.adaptiveRounds."""
     e = RenderExtensionB200()
     e.sType = STRUCTURE_TYPE_RENDER_EXTENSION_B200
     e.pNext = None
@@ -199,6 +207,19 @@ def make_extension(frames=1, accumulate=False, max_ray_depth=0, collect_stats=Fa
         e._view_array = (C.c_void_p * len(view_cameras))(*[c.h for c in view_cameras])  # kept alive with e
         e.viewCount = len(view_cameras)
         e.ppViewCameras = C.cast(e._view_array, C.c_void_p)
+    e.adaptiveError, e.adaptiveRoundFrames, e.adaptiveMaxFrames = adaptive_error, adaptive_round_frames, adaptive_max_frames
+    if pixel_frames is not None:
+        assert pixel_frames.dtype == np.uint32 and pixel_frames.flags["C_CONTIGUOUS"]
+        e._pixel_frames = pixel_frames  # kept alive with e
+        e.pPixelFrames = pixel_frames.ctypes.data
+    return e
+
+
+def scene_extension(scene_path):
+    """Host-only: the RenderExtensionB200 a .scene file gives the renderer (SceneParser::getRenderExtensionB200)"""
+    e = RenderExtensionB200()
+    if load().lth_scene_extension(scene_path.encode(), C.byref(e)) != 0:
+        raise RuntimeError("cannot parse scene file %s" % scene_path)
     return e
 
 

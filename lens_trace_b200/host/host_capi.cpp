@@ -169,4 +169,13 @@ int lth_run_scene_file(const char* scene_path, float* out, uint64_t out_bytes, u
   return 0;
 }
 
+// the RenderExtensionB200 a .scene file gives the renderer (no device needed); 0 on success
+int lth_scene_extension(const char* scene_path, void* ext_out) {
+  SceneParser parser(scene_path);
+  if (!parser.ok() || !ext_out) return -1;
+  RenderExtensionB200 ext = parser.getRenderExtensionB200();
+  memcpy(ext_out, &ext, sizeof ext);
+  return 0;
+}
+
 }  // extern "C"

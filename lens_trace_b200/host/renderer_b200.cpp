@@ -275,8 +275,32 @@ void RendererB200::renderCommon(const std::string& kernelFilePath, KernelMode ke
       memcpy(viewCameras.data() + (size_t)v * 28, ext->ppViewCameras[v]->getCameraBuffer(), 28);
     }
   }
+  const bool adaptive = ext && ext->adaptiveError > 0.0f;
+  if (adaptive) {  // the combinations lt_render_adaptive does not render: nothing is written
+    const char* why = !ext->accumulate ? "needs accumulate"
+                      : plugin >= 0    ? "renders the built-in kernels only"
+                      : views > 1      ? "renders one view"
+                      : ext->splitMode == LT_SPLIT_SAMPLES ? "divides the devices' work by rows, not samples"
+                                                           : nullptr;
+    if (why) {
+      printf("ERROR: RenderExtensionB200::adaptiveError %s\n", why);
+      return;
+    }
+  }
   int rc;
-  if (views > 1)
+  if (adaptive) {
+    lt_adaptive_params ap;
+    memset(&ap, 0, sizeof ap);
+    ap.struct_size = sizeof ap;
+    ap.target = ext->adaptiveError;
+    ap.round_frames = (int)ext->adaptiveRoundFrames;
+    const int round = ap.round_frames ? ap.round_frames : params.frames;
+    ap.max_frames = ext->adaptiveMaxFrames ? (int)ext->adaptiveMaxFrames : params.frames + 3 * round;  // INTEGRATION 5d
+    lt_adaptive_result res;
+    rc = lt_render_adaptive(useCtx, scene, camera->getCameraBuffer(), &params, &ap, (float*)pOutputBuffer,
+                            ext->pPixelFrames, &res);
+    if (rc == LT_OK) ext->adaptiveRounds = (uint32_t)res.rounds;
+  } else if (views > 1)
     rc = lt_render_views(useCtx, scene, viewCameras.data(), (int)views, &params, (float*)pOutputBuffer);
   else if (plugin >= 0 && ext)  // frames, accumulation and devices as the extension asks
     rc = lt_render_plugin_frames(useCtx, scene, camera->getCameraBuffer(), plugin, &params,

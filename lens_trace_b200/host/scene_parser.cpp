@@ -180,6 +180,9 @@ SceneParser::SceneParser(std::string filename) : parsedOk(false) {
       if (isStr(v, "samples")) rendererParsed.splitMode = 1;
       else if (isStr(v, "tiles")) rendererParsed.splitMode = 2;
     }
+    if (const JValue* v = r->get("adaptive_error")) rendererParsed.adaptiveError = (float)v->num;
+    if (const JValue* v = r->get("adaptive_round_frames")) rendererParsed.adaptiveRoundFrames = (uint32_t)v->num;
+    if (const JValue* v = r->get("adaptive_max_frames")) rendererParsed.adaptiveMaxFrames = (uint32_t)v->num;
   }
 
   if (const JValue* c = root.get("camera")) {
@@ -308,5 +311,8 @@ RenderExtensionB200 SceneParser::getRenderExtensionB200() {
   e.maxRayDepth = rendererParsed.maxRayDepth;
   e.deviceCount = rendererParsed.deviceCount;
   e.splitMode = rendererParsed.splitMode;
+  e.adaptiveError = rendererParsed.adaptiveError;
+  e.adaptiveRoundFrames = rendererParsed.adaptiveRoundFrames;
+  e.adaptiveMaxFrames = rendererParsed.adaptiveMaxFrames;
   return e;
 }
