@@ -109,6 +109,10 @@ typedef struct lt_render_params {
                              field is accepted and means LT_SPLIT_AUTO */
 } lt_render_params;
 
+/* Statistics of the context's last call (lt_last_stats).  Every field describes that call and reads 0 for what it did
+ * not measure: the counters (rays, node_tests, tri_tests) on a call without LT_FLAG_STATS, and kernel_ms and the
+ * per-kernel times on an asynchronous call (sync = 0 without LT_FLAG_STATS), which returns before its work is done.
+ * upload_ms instead describes the last lt_scene_upload or lt_scene_refit, and sm_count the device. */
 typedef struct lt_stats {
   uint64_t rays;        /* traversal calls (primary + shadow + extension + lens segments) */
   uint64_t node_tests;  /* boxes tested, reference traversal order */

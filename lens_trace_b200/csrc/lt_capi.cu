@@ -702,6 +702,27 @@ extern "C" int lt_debug_ctx_limits(lt_ctx* ctx, int threaded_max_nodes, int stre
   return LT_OK;
 }
 
+void lt_internal_stats_start(lt_ctx* ctx) {
+  lt_stats s = {};
+  s.sm_count = ctx->stats.sm_count;
+  s.upload_ms = ctx->stats.upload_ms;
+  ctx->stats = s;
+}
+
+// what one call adds to a sum of calls: counters, launches and per-kernel times (kernel_ms is the caller's to time)
+static void stats_add(lt_stats* sum, const lt_stats& s) {
+  sum->rays += s.rays;
+  sum->node_tests += s.node_tests;
+  sum->tri_tests += s.tri_tests;
+  sum->kernel_launches += s.kernel_launches;
+  sum->trace_ms += s.trace_ms;
+  sum->trace_launches += s.trace_launches;
+  sum->shade_ms += s.shade_ms;
+  sum->primary_shade_ms += s.primary_shade_ms;
+  sum->accumulate_ms += s.accumulate_ms;
+  sum->shade_launches += s.shade_launches;
+}
+
 int lt_internal_ensure_out(lt_ctx* ctx, size_t floats) {
   if (ctx->outFloats >= floats) return LT_OK;
   CK(ctx_grow(&ctx->dOut, &ctx->outFloats, floats, sizeof(float)));
@@ -715,6 +736,7 @@ int lt_internal_ensure_out(lt_ctx* ctx, size_t floats) {
 // list: the listed pixels of a masked call (lt_render_masked_device), or nullptr
 static int render_common(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, float* dOut, bool sync,
                          const RefCamera* cams = nullptr, int viewCount = 1, const LtList* list = nullptr) {
+  lt_internal_stats_start(ctx);
   CK(cudaSetDevice(ctx->device));
   const long long listed = list ? list->count : -1;
   LtPlan plan =
@@ -777,10 +799,10 @@ static int render_common(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, float*
   if (sync || stats) {
     CK(cudaStreamSynchronize(ctx->stream));
     CK(cudaEventElapsedTime(&ctx->stats.kernel_ms, ctx->ev0, ctx->ev1));
-    ctx->stats.trace_ms = wavefront ? 0.0f : ctx->stats.kernel_ms;
-    ctx->stats.trace_launches = wavefront ? 0 : launches;
-    ctx->stats.shade_ms = ctx->stats.primary_shade_ms = ctx->stats.accumulate_ms = 0.0f;
-    ctx->stats.shade_launches = 0;
+    if (!wavefront) {
+      ctx->stats.trace_ms = ctx->stats.kernel_ms;
+      ctx->stats.trace_launches = launches;
+    }
     for (int i = 0; i < tracePairs; i++) {
       float ms = 0.0f;
       cudaEventElapsedTime(&ms, ctx->traceEvents[2 * i], ctx->traceEvents[2 * i + 1]);
@@ -797,11 +819,6 @@ static int render_common(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, float*
         ctx->stats.accumulate_ms += ms;
       }
     }
-  } else {
-    ctx->stats.trace_ms = 0.0f;
-    ctx->stats.trace_launches = 0;
-    ctx->stats.shade_ms = ctx->stats.primary_shade_ms = ctx->stats.accumulate_ms = 0.0f;
-    ctx->stats.shade_launches = 0;
   }
   if (stats) {
     LtCounters h;
@@ -833,11 +850,7 @@ static const size_t kMaskListAt = 64, kListPad = 64;
 static int render_listed(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, int* dList, int count, float* dOut,
                          float* dM2, bool sync) {
   if (count == 0) {  // nothing to render: no pixel is written
-    const int sms = ctx->stats.sm_count;
-    const float uploadMs = ctx->stats.upload_ms;
-    ctx->stats = lt_stats{};
-    ctx->stats.sm_count = sms;
-    ctx->stats.upload_ms = uploadMs;
+    lt_internal_stats_start(ctx);
     return LT_OK;
   }
   const int extra = ctx->reverseList ? lt_launch_list_reverse(dList, count, ctx->stream) : 0;
@@ -902,7 +915,8 @@ static int adaptive_loop(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, const 
     count = lt_tile_rows_of(L.height, parts, part) * L.width;
   }
   CK(cudaGetLastError());
-  lt_stats sum = {};
+  lt_internal_stats_start(ctx);
+  lt_stats sum = ctx->stats;
   sum.kernel_launches = 1;
   int cur = 0, frames = L.frames, done = 0;
   bool waited = true;  // the device has finished every round counted in sum.kernel_ms
@@ -911,17 +925,7 @@ static int adaptive_loop(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, const 
     Lr.frames = frames;
     Lr.cam.frameCount = L.cam.frameCount + (unsigned)done;
     if (int rc = render_listed(ctx, scene, Lr, lists[cur], count, dOut, dM2, false)) return rc;
-    const lt_stats& r = ctx->stats;
-    sum.rays += r.rays;
-    sum.node_tests += r.node_tests;
-    sum.tri_tests += r.tri_tests;
-    sum.kernel_launches += r.kernel_launches;
-    sum.trace_ms += r.trace_ms;
-    sum.trace_launches += r.trace_launches;
-    sum.shade_ms += r.shade_ms;
-    sum.primary_shade_ms += r.primary_shade_ms;
-    sum.accumulate_ms += r.accumulate_ms;
-    sum.shade_launches += r.shade_launches;
+    stats_add(&sum, ctx->stats);
     res->rounds++;
     res->pixel_frames += (uint64_t)count * (uint64_t)frames;
     done += frames;
@@ -957,8 +961,6 @@ static int adaptive_loop(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, const 
     sum.kernel_ms += ms;
     waited = true;
   }
-  sum.sm_count = ctx->stats.sm_count;
-  sum.upload_ms = ctx->stats.upload_ms;
   if (!waited) sum.kernel_ms = 0.0f;  // not known before the work is done
   ctx->stats = sum;
   return LT_OK;
@@ -1066,16 +1068,8 @@ extern "C" int lt_debug_ctx_list_order(lt_ctx* ctx, int reversed) {
   return LT_OK;
 }
 
-int lt_internal_render_rows(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params,
-                            float* device_out, int fullHeight, int rowBlock, int rowStride, int rowPhase, int sync) {
-  LtLaunch L;
-  int rc = check_params(ctx, scene, camera28, params, &L);
-  if (rc != LT_OK) return rc;
-  L.fullHeight = fullHeight;
-  L.rowBlock = rowBlock;
-  L.rowStride = rowStride;
-  L.rowPhase = rowPhase;
-  return render_common(ctx, scene, L, device_out, sync != 0);
+int lt_internal_render(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, float* device_out) {
+  return render_common(ctx, scene, L, device_out, false);
 }
 
 // Result -> the caller's host buffer.  The reference hands render() a malloc'ed (pageable) pOutputBuffer
@@ -1178,17 +1172,15 @@ static int check_views(lt_ctx* ctx, const void* cameras28, int view_count, const
   return LT_OK;
 }
 
-int lt_internal_render_views(lt_ctx* ctx, lt_scene* scene, const RefCamera* cams, int count,
-                             const lt_render_params* params, float* host_out, int hostFirst, int hostStride) {
-  LtLaunch L;
-  int rc = check_params(ctx, scene, cams, params, &L);
-  if (rc != LT_OK) return rc;
+int lt_internal_render_views(lt_ctx* ctx, lt_scene* scene, LtLaunch L, const RefCamera* cams, int count,
+                             float* host_out, int hostFirst, int hostStride) {
+  L.cam = cams[0];  // the camera of a single view
   CK(cudaSetDevice(ctx->device));
   const size_t image = (size_t)L.width * L.height * L.depth, floats = image * (size_t)count;
   CK(ctx_grow(&ctx->dViews, &ctx->viewsFloats, floats, sizeof(float)));
   // every view accumulates from zero, as after lt_accum_reset
   CK(cudaMemsetAsync(ctx->dViews, 0, floats * sizeof(float), ctx->stream));
-  rc = render_common(ctx, scene, L, ctx->dViews, true, cams, count);
+  int rc = render_common(ctx, scene, L, ctx->dViews, true, cams, count);
   if (rc != LT_OK || !host_out) return rc;
   if (hostStride == 1)
     return lt_internal_download(ctx, host_out + (size_t)hostFirst * image, ctx->dViews, floats * sizeof(float));
@@ -1206,7 +1198,9 @@ extern "C" int lt_render_views(lt_ctx* ctx, lt_scene* scene, const void* cameras
     if (view_count == 1) return lt_multi_render(ctx, scene, cameras28, params, host_out, nullptr);
     return lt_multi_render_views(ctx, scene, cams.data(), view_count, params, host_out);
   }
-  return lt_internal_render_views(ctx, scene, cams.data(), view_count, params, host_out, 0, 1);
+  LtLaunch L;
+  if (int rc = check_params(ctx, scene, cameras28, params, &L)) return rc;
+  return lt_internal_render_views(ctx, scene, L, cams.data(), view_count, host_out, 0, 1);
 }
 
 extern "C" int lt_render_views_device(lt_ctx* ctx, lt_scene* scene, const void* cameras28, int view_count,
@@ -1240,6 +1234,7 @@ extern "C" int lt_plugin_load(lt_ctx* ctx, const char* kernel_file_path, int* ou
 
 int lt_internal_render_plugin(lt_ctx* ctx, lt_scene* scene, const RefCamera& cam, const lt_render_params& P,
                               const LtPluginRun& run, bool sync, const char* who) {
+  lt_internal_stats_start(ctx);
   CK(cudaSetDevice(ctx->device));
   LtPlugin* plugin = ctx->plugins[run.id];
   const bool cl = lt_plugin_is_opencl_c(plugin);
@@ -1292,9 +1287,6 @@ int lt_internal_render_plugin(lt_ctx* ctx, lt_scene* scene, const RefCamera& cam
   CK(cudaGetLastError());
   CK(cudaEventRecord(ctx->ev1, ctx->stream));
   ctx->stats.kernel_launches = launches;
-  ctx->stats.rays = ctx->stats.node_tests = ctx->stats.tri_tests = 0;
-  ctx->stats.trace_ms = ctx->stats.shade_ms = ctx->stats.primary_shade_ms = ctx->stats.accumulate_ms = 0.0f;
-  ctx->stats.trace_launches = ctx->stats.shade_launches = 0;
   if (sync) {
     CK(cudaStreamSynchronize(ctx->stream));
     CK(cudaEventElapsedTime(&ctx->stats.kernel_ms, ctx->ev0, ctx->ev1));

@@ -272,16 +272,18 @@ const std::vector<LtPlugin*>& lt_multi_plugins(const lt_ctx* ctx);  // device 0'
 void lt_multi_destroy(lt_ctx* ctx);
 int lt_multi_accum_reset(lt_ctx* ctx);
 int lt_internal_fail(lt_ctx* ctx, int code, const std::string& msg);  // sets the context's (and the thread's) last error
+// The start of every call's statistics: all of ctx->stats zero but sm_count and upload_ms (the last upload or refit).
+// A call then sets only what it measured.
+void lt_internal_stats_start(lt_ctx* ctx);
 int lt_internal_ensure_out(lt_ctx* ctx, size_t floats);
 // device -> the caller's host buffer on ctx's stream, synchronous (staged through pinned memory when pageable)
 int lt_internal_download(lt_ctx* ctx, float* host_out, const float* dSrc, size_t bytes);
-// one device's share of a render call: like lt_render_device, with the row window of a tile split
-int lt_internal_render_rows(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params,
-                            float* device_out, int fullHeight, int rowBlock, int rowStride, int rowPhase, int sync);
-// lt_render_views on one device: view k (camera cams[k]) into the context's view buffer, from zero, and then (host_out
-// != NULL) to host_out + (hostFirst + k * hostStride) * W * H * depth
-int lt_internal_render_views(lt_ctx* ctx, lt_scene* scene, const RefCamera* cams, int count,
-                             const lt_render_params* params, float* host_out, int hostFirst, int hostStride);
+// one device's share of a render call (L checked, camera and row window included): lt_render_device, asynchronous
+int lt_internal_render(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, float* device_out);
+// lt_render_views on one device (L checked; its camera is not used): view k (camera cams[k]) into the context's view
+// buffer, from zero, and then (host_out != NULL) to host_out + (hostFirst + k * hostStride) * W * H * depth
+int lt_internal_render_views(lt_ctx* ctx, lt_scene* scene, LtLaunch L, const RefCamera* cams, int count,
+                             float* host_out, int hostFirst, int hostStride);
 int lt_multi_render_views(lt_ctx* ctx, lt_scene* scene, const RefCamera* cams, int count, const lt_render_params* params,
                           float* host_out);
 // lt_render_adaptive's host form on one device (arguments checked; L.cam is the camera): the rows of part `part` of a

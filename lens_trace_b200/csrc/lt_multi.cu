@@ -21,6 +21,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <string>
 #include <thread>
 #include <vector>
@@ -167,6 +168,47 @@ void lt_multi_destroy(lt_ctx* ctx) {
   ctx->group = nullptr;
 }
 
+// The one place that runs work on the devices of a group: fn(k) for the devices k = 0 .. n-1, each on a host thread of
+// its own, joined before it returns.  Every device's statistics start first, so that a device with no share in the
+// call reports zeros.  Returns LT_OK, or the code of the lowest-numbered device that failed, with that device's message
+// copied to the group context.
+template <class Fn>
+static int fan_out(lt_ctx* ctx, int n, Fn fn) {
+  LtGroup* g = ctx->group;
+  for (lt_ctx* c : g->ctx) lt_internal_stats_start(c);
+  std::vector<int> rcs(n, LT_OK);
+  std::vector<std::thread> workers;
+  for (int k = 0; k < n; k++) workers.emplace_back([&, k]() { rcs[k] = fn(k); });
+  for (std::thread& t : workers) t.join();
+  for (int k = 0; k < n; k++)
+    if (rcs[k] != LT_OK) return lt_internal_fail(ctx, rcs[k], lt_last_error(g->ctx[k]));
+  return LT_OK;
+}
+
+// c's device made current on the calling thread, or LT_ERR_CUDA with c's message
+static int use_device(lt_ctx* c) {
+  const cudaError_t e = cudaSetDevice(c->device);
+  if (e == cudaSuccess) return LT_OK;
+  return lt_internal_fail(c, LT_ERR_CUDA, std::string("cudaSetDevice: ") + cudaGetErrorString(e));
+}
+
+// upload and refit: the slowest device's time
+static void merge_upload_ms(lt_ctx* ctx) {
+  ctx->stats.upload_ms = 0.0f;
+  for (const lt_ctx* c : ctx->group->ctx) ctx->stats.upload_ms = std::max(ctx->stats.upload_ms, c->stats.upload_ms);
+}
+
+// A render call's statistics: the slowest device's kernel time and every device's launches.  Leaves device 0 current
+// on the calling thread.
+static void merge_render_stats(lt_ctx* ctx) {
+  lt_internal_stats_start(ctx);
+  for (const lt_ctx* c : ctx->group->ctx) {
+    ctx->stats.kernel_ms = std::max(ctx->stats.kernel_ms, c->stats.kernel_ms);
+    ctx->stats.kernel_launches += c->stats.kernel_launches;
+  }
+  cudaSetDevice(ctx->group->ctx[0]->device);
+}
+
 int lt_multi_scene_upload(lt_ctx* ctx, const void* nodes, uint64_t node_bytes, const void* primitives,
                           uint64_t primitive_bytes, const void* materials, uint64_t material_bytes,
                           const void* light_container, uint64_t light_bytes, lt_scene** out_scene) {
@@ -174,44 +216,27 @@ int lt_multi_scene_upload(lt_ctx* ctx, const void* nodes, uint64_t node_bytes, c
   *out_scene = nullptr;
   lt_scene* s = new lt_scene();
   s->parts.resize(g->ctx.size(), nullptr);
-  std::vector<int> rcs(g->ctx.size(), LT_OK);
-  std::vector<std::thread> workers;
-  for (size_t k = 0; k < g->ctx.size(); k++)
-    workers.emplace_back([&, k]() {
-      rcs[k] = lt_scene_upload(g->ctx[k], nodes, node_bytes, primitives, primitive_bytes, materials, material_bytes,
-                               light_container, light_bytes, &s->parts[k]);
-    });
-  for (std::thread& t : workers) t.join();
-  float ms = 0.0f;
-  for (size_t k = 0; k < g->ctx.size(); k++)
-    if (g->ctx[k]->stats.upload_ms > ms) ms = g->ctx[k]->stats.upload_ms;
-  ctx->stats.upload_ms = ms;
-  for (size_t k = 0; k < g->ctx.size(); k++)
-    if (rcs[k] != LT_OK) {
-      std::string why = lt_last_error(g->ctx[k]);
-      for (size_t j = 0; j < g->ctx.size(); j++)
-        if (s->parts[j]) lt_scene_release(g->ctx[j], s->parts[j]);
-      delete s;
-      return lt_internal_fail(ctx, rcs[k], why);
-    }
+  const int rc = fan_out(ctx, (int)g->ctx.size(), [&](int k) {
+    return lt_scene_upload(g->ctx[k], nodes, node_bytes, primitives, primitive_bytes, materials, material_bytes,
+                           light_container, light_bytes, &s->parts[k]);
+  });
+  merge_upload_ms(ctx);
+  if (rc != LT_OK) {
+    for (size_t j = 0; j < g->ctx.size(); j++)
+      if (s->parts[j]) lt_scene_release(g->ctx[j], s->parts[j]);
+    delete s;
+    return rc;
+  }
   *out_scene = s;
   return LT_OK;
 }
 
 int lt_multi_scene_refit(lt_ctx* ctx, lt_scene* scene, const void* primitives) {
   LtGroup* g = ctx->group;
-  std::vector<int> rcs(g->ctx.size(), LT_OK);
-  std::vector<std::thread> workers;
-  for (size_t k = 0; k < g->ctx.size(); k++)
-    workers.emplace_back([&, k]() { rcs[k] = lt_internal_refit(g->ctx[k], scene->parts[k], primitives); });
-  for (std::thread& t : workers) t.join();
-  float ms = 0.0f;
-  for (size_t k = 0; k < g->ctx.size(); k++)
-    if (g->ctx[k]->stats.upload_ms > ms) ms = g->ctx[k]->stats.upload_ms;
-  ctx->stats.upload_ms = ms;
-  for (size_t k = 0; k < g->ctx.size(); k++)
-    if (rcs[k] != LT_OK) return lt_internal_fail(ctx, rcs[k], lt_last_error(g->ctx[k]));
-  return LT_OK;
+  const int rc = fan_out(ctx, (int)g->ctx.size(),
+                         [&](int k) { return lt_internal_refit(g->ctx[k], scene->parts[k], primitives); });
+  merge_upload_ms(ctx);
+  return rc;
 }
 
 void lt_multi_scene_release(lt_ctx* ctx, lt_scene* scene) {
@@ -234,25 +259,21 @@ int lt_multi_accum_reset(lt_ctx* ctx) {
 // device's context holds the plug-in under the same id.
 int lt_multi_plugin_load(lt_ctx* ctx, const LtPluginImage& img, int* out_plugin_id) {
   LtGroup* g = ctx->group;
-  const size_t G = g->ctx.size();
+  const int G = (int)g->ctx.size();
   std::vector<LtPlugin*> loaded(G, nullptr);
-  std::vector<std::string> errs(G);
-  std::vector<std::thread> workers;
-  for (size_t k = 0; k < G; k++)
-    workers.emplace_back([&, k]() {
-      if (cudaSetDevice(g->ctx[k]->device) != cudaSuccess || cudaFree(0) != cudaSuccess) {
-        errs[k] = "cannot make device " + std::to_string(g->ctx[k]->device) + " current";
-        return;
-      }
-      loaded[k] = lt_plugin_module_load(img, &errs[k]);
-    });
-  for (std::thread& t : workers) t.join();
-  for (size_t k = 0; k < G; k++)
-    if (!loaded[k]) {
-      for (LtPlugin* p : loaded) lt_plugin_free(p);
-      return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED, "lt_plugin_load: " + errs[k]);
-    }
-  for (size_t k = 0; k < G; k++) g->ctx[k]->plugins.push_back(loaded[k]);
+  const int rc = fan_out(ctx, G, [&](int k) {
+    std::string err;
+    if (cudaSetDevice(g->ctx[k]->device) != cudaSuccess || cudaFree(0) != cudaSuccess)
+      err = "cannot make device " + std::to_string(g->ctx[k]->device) + " current";
+    else
+      loaded[k] = lt_plugin_module_load(img, &err);
+    return loaded[k] ? LT_OK : lt_internal_fail(g->ctx[k], LT_ERR_UNSUPPORTED, "lt_plugin_load: " + err);
+  });
+  if (rc != LT_OK) {
+    for (LtPlugin* p : loaded) lt_plugin_free(p);
+    return rc;
+  }
+  for (int k = 0; k < G; k++) g->ctx[k]->plugins.push_back(loaded[k]);
   *out_plugin_id = (int)g->ctx[0]->plugins.size() - 1;
   return LT_OK;
 }
@@ -370,33 +391,54 @@ extern "C" int lt_debug_tile_rows(int height, int devices, int device, int32_t* 
   return rows;
 }
 
+// The checks of a multi-GPU render call, all before any device works: the arguments, the scene, and every check of the
+// single-GPU call (lt_params_to_launch, under `who`).  Out: the normalised parameters and their launch, camera
+// included.  Each entry point adds its own split_mode rules.
+static int render_prologue(lt_ctx* ctx, const lt_scene* scene, const void* camera28, const lt_render_params* params,
+                           const char* who, lt_render_params* P, LtLaunch* L) {
+  const std::string w = std::string(who) + ": ";
+  if (!scene || !camera28 || !params) return lt_internal_fail(ctx, LT_ERR_INVALID, w + "NULL argument");
+  if (scene->parts.size() != ctx->group->ctx.size())
+    return lt_internal_fail(ctx, LT_ERR_INVALID, w + "the scene was not uploaded through this multi-GPU context");
+  if (int rc = lt_params_normalise(ctx, params, w, P)) return rc;
+  if (int rc = lt_params_to_launch(ctx, P, L, who)) return rc;
+  memcpy(&L->cam, camera28, sizeof(RefCamera));
+  if (P->flags & LT_FLAG_STATS)
+    return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED, w + "LT_FLAG_STATS counts on a single-GPU context");
+  return LT_OK;
+}
+
 int lt_multi_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt_render_params* params, float* host_out,
                     const LtPluginRun* run) {
   LtGroup* g = ctx->group;
-  const std::string who = run ? "lt_render_plugin_frames: " : "lt_render: ";
-  if (!scene || !camera28 || !params) return lt_internal_fail(ctx, LT_ERR_INVALID, who + "NULL argument");
-  if (scene->parts.size() != g->ctx.size())
-    return lt_internal_fail(ctx, LT_ERR_INVALID, who + "the scene was not uploaded through this multi-GPU context");
+  const char* who = run ? "lt_render_plugin_frames" : "lt_render";
+  const std::string w = std::string(who) + ": ";
   lt_render_params P;
-  if (int rc = lt_params_normalise(ctx, params, who, &P)) return rc;
-  if (P.width <= 0 || P.height <= 0 || P.depth < 3 || P.frames < 1)
-    return lt_internal_fail(ctx, LT_ERR_INVALID, who + "width/height must be > 0, depth >= 3, frames >= 1");
-  if (P.flags & LT_FLAG_STATS)
-    return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED, who + "LT_FLAG_STATS counts on a single-GPU context");
+  LtLaunch L;
+  if (int rc = render_prologue(ctx, scene, camera28, params, who, &P, &L)) return rc;
   const int G = (int)g->ctx.size();
   int split = P.split_mode;
   // a plug-in derives its pixel from blockIdx / get_global_id: it cannot be given a subset of the rows
   if (run && split == LT_SPLIT_TILES)
-    return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED, who + "a plug-in cannot render a tile split (use LT_SPLIT_SAMPLES)");
+    return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED, w + "a plug-in cannot render a tile split (use LT_SPLIT_SAMPLES)");
   if (split == LT_SPLIT_AUTO)
-    split = (run || (P.frames >= 2 && P.accum_mode != LT_ACCUM_NONE)) ? LT_SPLIT_SAMPLES : LT_SPLIT_TILES;
-  if (split == LT_SPLIT_SAMPLES && P.accum_mode == LT_ACCUM_NONE)
+    split = (run || (L.frames >= 2 && L.accumMode != LT_ACCUM_NONE)) ? LT_SPLIT_SAMPLES : LT_SPLIT_TILES;
+  if (split == LT_SPLIT_SAMPLES && L.accumMode == LT_ACCUM_NONE)
     return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED,
-                            who + "a sample split needs an accumulating call (LT_ACCUM_NONE keeps only the last frame)");
-  if (split != LT_SPLIT_SAMPLES && split != LT_SPLIT_TILES) return lt_internal_fail(ctx, LT_ERR_INVALID, who + "bad split_mode");
-  RefCamera cam;
-  memcpy(&cam, camera28, sizeof cam);
-  const size_t fullFloats = (size_t)P.width * P.height * P.depth;
+                            w + "a sample split needs an accumulating call (LT_ACCUM_NONE keeps only the last frame)");
+  if (split != LT_SPLIT_SAMPLES && split != LT_SPLIT_TILES) return lt_internal_fail(ctx, LT_ERR_INVALID, w + "bad split_mode");
+  const bool mean = L.accumMode == LT_ACCUM_RUNNING_MEAN;
+  const size_t fullFloats = (size_t)L.width * L.height * L.depth;
+  bool useNccl = false;
+  if (split == LT_SPLIT_SAMPLES) {
+    if (mean && L.frameStride != 1u)
+      return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED, w + "a multi-GPU running mean needs frame_stride 1");
+    std::string why;
+    const char* ex = getenv("LT_MULTI_EXCHANGE");
+    useNccl = !(ex && strcmp(ex, "p2p") == 0) && ensure_nccl(g, &why);
+    if (!useNccl && !ensure_peers(g, fullFloats, &why))
+      return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED, w + "no way to combine the devices' accumulators: " + why);
+  }
   // the devices' accumulators are only comparable while split and size stay the same
   if (g->lastSplit != split || g->lastFloats != (long long)fullFloats) {
     int rc = lt_multi_accum_reset(ctx);
@@ -404,82 +446,68 @@ int lt_multi_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt
     g->lastSplit = split;
     g->lastFloats = (long long)fullFloats;
   }
-  std::vector<int> rcs(G, LT_OK);
-  std::vector<std::thread> workers;
-  const uint32_t stride = P.frame_stride ? P.frame_stride : 1u;
 
   if (split == LT_SPLIT_TILES) {
-    std::vector<int> rows(G);
-    for (int k = 0; k < G; k++) rows[k] = lt_tile_rows_of(P.height, G, k);
-    const size_t rowBytes = (size_t)P.width * P.depth * sizeof(float);
-    for (int k = 0; k < G; k++)
-      workers.emplace_back([&, k]() {
-        lt_ctx* c = g->ctx[k];
-        if (rows[k] == 0) return;
-        if (cudaSetDevice(c->device) != cudaSuccess) { rcs[k] = LT_ERR_CUDA; return; }
-        rcs[k] = lt_internal_ensure_out(c, (size_t)P.width * rows[k] * P.depth);
-        if (rcs[k] != LT_OK) return;
-        lt_render_params Pk = P;
-        Pk.height = rows[k];
-        Pk.split_mode = 0;
-        rcs[k] = lt_internal_render_rows(c, scene->parts[k], &cam, &Pk, c->dOut, P.height, LT_TILE_ROWS, G, k, 0);
-        if (rcs[k] != LT_OK || !host_out) return;
-        cudaError_t e = lt_copy_row_blocks(host_out, c->dOut, LT_TILE_ROWS * rowBytes, rowBytes, rows[k], G, k, c->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-        if (e != cudaSuccess) rcs[k] = lt_internal_fail(c, LT_ERR_CUDA, std::string("tile copy: ") + cudaGetErrorString(e));
-      });
-    for (std::thread& t : workers) t.join();
-    if (!host_out)
-      for (int k = 0; k < G; k++) {
-        cudaSetDevice(g->ctx[k]->device);
-        cudaStreamSynchronize(g->ctx[k]->stream);
-      }
+    const size_t rowBytes = (size_t)L.width * L.depth * sizeof(float);
+    const int rc = fan_out(ctx, G, [&](int k) -> int {
+      lt_ctx* c = g->ctx[k];
+      const int rows = lt_tile_rows_of(L.height, G, k);
+      if (rows == 0) return LT_OK;
+      if (int e = use_device(c)) return e;
+      if (int e = lt_internal_ensure_out(c, (size_t)L.width * rows * L.depth)) return e;
+      LtLaunch Lk = L;  // every G-th block of LT_TILE_ROWS rows from block k
+      Lk.height = rows;
+      Lk.rowBlock = LT_TILE_ROWS;
+      Lk.rowStride = G;
+      Lk.rowPhase = k;
+      if (int e = lt_internal_render(c, scene->parts[k], Lk, c->dOut)) return e;
+      if (!host_out) return LT_OK;
+      cudaError_t e = lt_copy_row_blocks(host_out, c->dOut, LT_TILE_ROWS * rowBytes, rowBytes, rows, G, k, c->stream);
+      if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+      return e == cudaSuccess ? LT_OK : lt_internal_fail(c, LT_ERR_CUDA, std::string("tile copy: ") + cudaGetErrorString(e));
+    });
+    if (rc != LT_OK) return rc;
   } else {
     // ---- sample split ----
-    if (P.accum_mode == LT_ACCUM_RUNNING_MEAN && stride != 1u)
-      return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED, who + "a multi-GPU running mean needs frame_stride 1");
-    const bool mean = P.accum_mode == LT_ACCUM_RUNNING_MEAN;
     // running mean: new = old * fc/(fc+F) + sum(samples)/(fc+F)  (fc = frames already in the accumulator; 0 discards it,
     // like frameCount == 0 in accumulator.frag:10-19)
-    const double total = (double)cam.frameCount + (double)P.frames;
-    const float weight = mean ? (float)(1.0 / total) : P.accum_weight;
-    const float keep = mean ? (float)((double)cam.frameCount / total) : 1.0f;
-    std::string why;
-    const char* ex = getenv("LT_MULTI_EXCHANGE");
-    bool useNccl = !(ex && strcmp(ex, "p2p") == 0) && ensure_nccl(g, &why);
-    if (!useNccl && !ensure_peers(g, fullFloats, &why))
-      return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED, who + "no way to combine the devices' accumulators: " + why);
-    for (int k = 0; k < G; k++)
-      workers.emplace_back([&, k]() {
-        lt_ctx* c = g->ctx[k];
-        if (cudaSetDevice(c->device) != cudaSuccess) { rcs[k] = LT_ERR_CUDA; return; }
-        rcs[k] = lt_internal_ensure_out(c, fullFloats);
-        if (rcs[k] != LT_OK) return;
-        // device 0 carries the accumulator that was there before this call, the others start from zero
-        if (k == 0) {
-          if (keep == 0.0f) cudaMemsetAsync(c->dOut, 0, fullFloats * sizeof(float), c->stream);
-          else if (keep != 1.0f) k_scale<<<c->stats.sm_count * 8, 256, 0, c->stream>>>(c->dOut, fullFloats, keep);
-        } else {
-          cudaMemsetAsync(c->dOut, 0, fullFloats * sizeof(float), c->stream);
-        }
-        const int nk = (P.frames - k + G - 1) / G;  // frames k, k+G, ... < P.frames
-        if (nk > 0 && k < P.frames) {
+    const double total = (double)L.cam.frameCount + (double)L.frames;
+    const float weight = mean ? (float)(1.0 / total) : L.accumWeight;
+    const float keep = mean ? (float)((double)L.cam.frameCount / total) : 1.0f;
+    const int rc = fan_out(ctx, G, [&](int k) -> int {
+      lt_ctx* c = g->ctx[k];
+      if (int e = use_device(c)) return e;
+      if (int e = lt_internal_ensure_out(c, fullFloats)) return e;
+      // device 0 carries the accumulator that was there before this call, the others start from zero
+      if (k == 0) {
+        if (keep == 0.0f) cudaMemsetAsync(c->dOut, 0, fullFloats * sizeof(float), c->stream);
+        else if (keep != 1.0f) k_scale<<<c->stats.sm_count * 8, 256, 0, c->stream>>>(c->dOut, fullFloats, keep);
+      } else {
+        cudaMemsetAsync(c->dOut, 0, fullFloats * sizeof(float), c->stream);
+      }
+      int e = LT_OK;
+      if (k < L.frames) {  // frames k, k+G, ... < L.frames, a weighted sum
+        LtLaunch Lk = L;
+        Lk.frames = (L.frames - k + G - 1) / G;
+        Lk.frameStride = L.frameStride * (uint32_t)G;
+        Lk.accumMode = LT_ACCUM_WEIGHTED_SUM;
+        Lk.accumWeight = weight;
+        Lk.cam.frameCount = L.cam.frameCount + (uint32_t)k * L.frameStride;
+        if (run) {
           lt_render_params Pk = P;
-          Pk.frames = nk;
-          Pk.frame_stride = stride * (uint32_t)G;
-          Pk.accum_mode = LT_ACCUM_WEIGHTED_SUM;
+          Pk.frames = Lk.frames;
+          Pk.frame_stride = Lk.frameStride;
+          Pk.accum_mode = Lk.accumMode;
           Pk.accum_weight = weight;
-          Pk.split_mode = 0;
-          RefCamera ck = cam;
-          ck.frameCount = cam.frameCount + (uint32_t)k * stride;
-          rcs[k] = run ? lt_internal_render_plugin(c, scene->parts[k], ck, Pk, *run, false, "lt_render_plugin_frames")
-                       : lt_internal_render_rows(c, scene->parts[k], &ck, &Pk, c->dOut, P.height, P.height, 1, 0, 0);
+          e = lt_internal_render_plugin(c, scene->parts[k], Lk.cam, Pk, *run, false, who);
+        } else {
+          e = lt_internal_render(c, scene->parts[k], Lk, c->dOut);
         }
-        cudaEventRecord(g->rendered[k], c->stream);
-      });
-    for (std::thread& t : workers) t.join();
-    for (int k = 0; k < G; k++)
-      if (rcs[k] != LT_OK) return lt_internal_fail(ctx, rcs[k], lt_last_error(g->ctx[k]));
+      }
+      cudaEventRecord(g->rendered[k], c->stream);
+      return e;
+    });
+    if (rc != LT_OK) return rc;
     // ---- the exchange step: one all-reduce(sum) of W*H*depth floats ----
     if (useNccl) {
       g_nccl.groupStart();
@@ -514,30 +542,21 @@ int lt_multi_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt
     }
     lt_ctx* c0 = g->ctx[0];
     cudaSetDevice(c0->device);
-    if (host_out) {
-      int rc = lt_internal_download(c0, host_out, c0->dOut, fullFloats * sizeof(float));
-      if (rc != LT_OK) rcs[0] = rc;
-    }
-    for (int k = 0; k < G; k++) {
-      cudaSetDevice(g->ctx[k]->device);
-      cudaError_t e = cudaStreamSynchronize(g->ctx[k]->stream);
-      if (e != cudaSuccess) rcs[k] = lt_internal_fail(g->ctx[k], LT_ERR_CUDA, std::string("multi-GPU render: ") + cudaGetErrorString(e));
-    }
+    if (host_out)
+      if (int e = lt_internal_download(c0, host_out, c0->dOut, fullFloats * sizeof(float)))
+        return lt_internal_fail(ctx, e, lt_last_error(c0));
   }
-  for (int k = 0; k < G; k++)
-    if (rcs[k] != LT_OK) return lt_internal_fail(ctx, rcs[k], lt_last_error(g->ctx[k]));
-  // statistics of the call: the slowest device's kernels, all devices' launches
-  ctx->stats.kernel_ms = 0.0f;
-  ctx->stats.kernel_launches = 0;
-  for (int k = 0; k < G; k++) {
-    lt_ctx* c = g->ctx[k];
-    float ms = 0.0f;
+  // the devices rendered asynchronously: wait for each, then time the kernels of those that rendered
+  for (lt_ctx* c : g->ctx) {
     cudaSetDevice(c->device);
-    if (cudaEventElapsedTime(&ms, c->ev0, c->ev1) == cudaSuccess && ms > ctx->stats.kernel_ms) ctx->stats.kernel_ms = ms;
+    const cudaError_t e = cudaStreamSynchronize(c->stream);
+    if (e != cudaSuccess)
+      return lt_internal_fail(ctx, LT_ERR_CUDA, std::string("multi-GPU render: ") + cudaGetErrorString(e));
+    float ms = 0.0f;
+    if (c->stats.kernel_launches > 0 && cudaEventElapsedTime(&ms, c->ev0, c->ev1) == cudaSuccess) c->stats.kernel_ms = ms;
     cudaGetLastError();
-    ctx->stats.kernel_launches += c->stats.kernel_launches;
   }
-  cudaSetDevice(g->ctx[0]->device);
+  merge_render_stats(ctx);
   return LT_OK;
 }
 
@@ -546,37 +565,20 @@ int lt_multi_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt
 int lt_multi_render_views(lt_ctx* ctx, lt_scene* scene, const RefCamera* cams, int count, const lt_render_params* params,
                           float* host_out) {
   LtGroup* g = ctx->group;
-  const std::string who = "lt_render_views: ";
-  if (!scene || !params) return lt_internal_fail(ctx, LT_ERR_INVALID, who + "NULL argument");
-  if (scene->parts.size() != g->ctx.size())
-    return lt_internal_fail(ctx, LT_ERR_INVALID, who + "the scene was not uploaded through this multi-GPU context");
   lt_render_params P;
-  if (int rc = lt_params_normalise(ctx, params, who, &P)) return rc;
+  LtLaunch L;
+  if (int rc = render_prologue(ctx, scene, cams, params, "lt_render_views", &P, &L)) return rc;
   if (P.split_mode != LT_SPLIT_AUTO)
-    return lt_internal_fail(ctx, LT_ERR_INVALID, who + "views are dealt to the devices whole: split_mode must be LT_SPLIT_AUTO");
-  if (P.flags & LT_FLAG_STATS)
-    return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED, who + "LT_FLAG_STATS counts on a single-GPU context");
+    return lt_internal_fail(ctx, LT_ERR_INVALID,
+                            "lt_render_views: views are dealt to the devices whole: split_mode must be LT_SPLIT_AUTO");
   const int G = (int)g->ctx.size();
-  std::vector<int> rcs(G, LT_OK);
-  std::vector<std::thread> workers;
-  for (int k = 0; k < G && k < count; k++)
-    workers.emplace_back([&, k]() {
-      std::vector<RefCamera> mine;
-      for (int v = k; v < count; v += G) mine.push_back(cams[v]);
-      rcs[k] = lt_internal_render_views(g->ctx[k], scene->parts[k], mine.data(), (int)mine.size(), &P, host_out, k, G);
-    });
-  for (std::thread& t : workers) t.join();
-  for (int k = 0; k < G; k++)
-    if (rcs[k] != LT_OK) return lt_internal_fail(ctx, rcs[k], lt_last_error(g->ctx[k]));
-  // statistics of the call: the slowest device's kernels, all devices' launches
-  ctx->stats.kernel_ms = 0.0f;
-  ctx->stats.kernel_launches = 0;
-  for (int k = 0; k < G && k < count; k++) {
-    const lt_ctx* c = g->ctx[k];
-    if (c->stats.kernel_ms > ctx->stats.kernel_ms) ctx->stats.kernel_ms = c->stats.kernel_ms;
-    ctx->stats.kernel_launches += c->stats.kernel_launches;
-  }
-  cudaSetDevice(g->ctx[0]->device);
+  const int rc = fan_out(ctx, std::min(G, count), [&](int k) {
+    std::vector<RefCamera> mine;
+    for (int v = k; v < count; v += G) mine.push_back(cams[v]);
+    return lt_internal_render_views(g->ctx[k], scene->parts[k], L, mine.data(), (int)mine.size(), host_out, k, G);
+  });
+  if (rc != LT_OK) return rc;
+  merge_render_stats(ctx);
   return LT_OK;
 }
 
@@ -588,47 +590,28 @@ int lt_multi_render_adaptive(lt_ctx* ctx, lt_scene* scene, const void* camera28,
                              const lt_adaptive_params* aparams, float* host_out, uint32_t* host_frames,
                              lt_adaptive_result* out_result) {
   LtGroup* g = ctx->group;
-  const std::string who = "lt_render_adaptive: ";
-  if (!scene || !camera28 || !params) return lt_internal_fail(ctx, LT_ERR_INVALID, who + "NULL argument");
-  if (scene->parts.size() != g->ctx.size())
-    return lt_internal_fail(ctx, LT_ERR_INVALID, who + "the scene was not uploaded through this multi-GPU context");
+  const char* who = "lt_render_adaptive";
   lt_render_params P;
-  if (int rc = lt_params_normalise(ctx, params, who, &P)) return rc;
-  if (P.split_mode != LT_SPLIT_AUTO && P.split_mode != LT_SPLIT_TILES)
-    return lt_internal_fail(ctx, LT_ERR_INVALID, who + "the devices share the image by rows: split_mode must be LT_SPLIT_AUTO or LT_SPLIT_TILES");
-  P.split_mode = LT_SPLIT_AUTO;
-  // every check of the single-GPU call, before any device works
   LtLaunch L;
-  if (int rc = lt_params_to_launch(ctx, &P, &L, "lt_render_adaptive")) return rc;
-  memcpy(&L.cam, camera28, sizeof(RefCamera));
+  if (int rc = render_prologue(ctx, scene, camera28, params, who, &P, &L)) return rc;
+  if (P.split_mode != LT_SPLIT_AUTO && P.split_mode != LT_SPLIT_TILES)
+    return lt_internal_fail(ctx, LT_ERR_INVALID, std::string(who) + ": the devices share the image by rows: split_mode "
+                                                 "must be LT_SPLIT_AUTO or LT_SPLIT_TILES");
   LtAdaptive A;
-  if (int rc = lt_adaptive_check(ctx, L, aparams, "lt_render_adaptive", &A)) return rc;
-  if (P.flags & LT_FLAG_STATS)
-    return lt_internal_fail(ctx, LT_ERR_UNSUPPORTED, who + "LT_FLAG_STATS counts on a single-GPU context");
+  if (int rc = lt_adaptive_check(ctx, L, aparams, who, &A)) return rc;
   const int G = (int)g->ctx.size();
-  std::vector<int> rcs(G, LT_OK);
   std::vector<lt_adaptive_result> res(G, lt_adaptive_result{});
-  std::vector<std::thread> workers;
-  for (int k = 0; k < G; k++)
-    workers.emplace_back([&, k]() {
-      rcs[k] = lt_internal_render_adaptive(g->ctx[k], scene->parts[k], L, A, host_out, host_frames, G, k, &res[k]);
-    });
-  for (std::thread& t : workers) t.join();
-  for (int k = 0; k < G; k++)
-    if (rcs[k] != LT_OK) return lt_internal_fail(ctx, rcs[k], lt_last_error(g->ctx[k]));
+  const int rc = fan_out(ctx, G, [&](int k) {
+    return lt_internal_render_adaptive(g->ctx[k], scene->parts[k], L, A, host_out, host_frames, G, k, &res[k]);
+  });
+  if (rc != LT_OK) return rc;
   lt_adaptive_result r = {};
-  ctx->stats.kernel_ms = 0.0f;
-  ctx->stats.kernel_launches = 0;
   for (int k = 0; k < G; k++) {
     if (res[k].rounds > r.rounds) r.rounds = res[k].rounds;
     r.pixel_frames += res[k].pixel_frames;
     r.pixels_unconverged += res[k].pixels_unconverged;
-    // statistics of the call: the slowest device's kernels, all devices' launches
-    const lt_ctx* c = g->ctx[k];
-    if (c->stats.kernel_ms > ctx->stats.kernel_ms) ctx->stats.kernel_ms = c->stats.kernel_ms;
-    ctx->stats.kernel_launches += c->stats.kernel_launches;
   }
   if (out_result) *out_result = r;
-  cudaSetDevice(g->ctx[0]->device);
+  merge_render_stats(ctx);
   return LT_OK;
 }
