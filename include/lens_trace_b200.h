@@ -367,6 +367,12 @@ int lt_debug_gather_peak(lt_ctx* ctx, uint64_t table_bytes, int dependent, int i
  * in the order of its local rows; returns their number (out_rows may be NULL to ask for it), negative on bad
  * arguments.  For tests of the partition on a machine without a GPU. */
 int lt_debug_tile_rows(int height, int devices, int device, int32_t* out_rows, int capacity);
+/* Test hook: a multi-GPU context of `members` (2..16) members that all render on device device_ordinal -- the group
+ * lt_ctx_create_multi builds, each member an ordinary single-GPU context with its own stream, buffers, scene copy and
+ * host thread -- so that the splits, the exchange kernel and the row copies run on a machine with one GPU.  Its sample
+ * split always combines the members' accumulators with the library's own exchange kernel (no NCCL, no peer mapping).
+ * Anything else than 2..16 members: LT_ERR_INVALID. */
+int lt_debug_ctx_create_shared(int device_ordinal, int members, lt_ctx** out_ctx);
 
 /* Host-only (no device needed): the threaded form of a reference node array that lt_scene_upload builds for
  * small trees -- 8 copies of node_count 32-byte records {lo.x lo.y lo.z hi.x | hi.y hi.z link skip}, copy o in

@@ -24,6 +24,7 @@ SYMBOLS = [
     "lt_debug_plan_views", "lt_scene_refit", "lt_scene_refit_device", "lt_debug_scene_bytes",
     "lt_render_masked_device", "lt_debug_plan_masked", "lt_debug_ctx_list_order", "lt_render_adaptive",
     "lt_render_adaptive_device", "lt_debug_adaptive_rounds", "lt_debug_ctx_adaptive_part",
+    "lt_debug_ctx_create_shared",
 ]
 
 
@@ -79,6 +80,7 @@ def load():
     lib.lt_api_version.restype = C.c_int
     lib.lt_ctx_create.argtypes = [C.c_int, C.POINTER(C.c_void_p)]
     lib.lt_ctx_create_multi.argtypes = [C.POINTER(C.c_int), C.c_int, C.POINTER(C.c_void_p)]
+    lib.lt_debug_ctx_create_shared.argtypes = [C.c_int, C.c_int, C.POINTER(C.c_void_p)]
     lib.lt_ctx_device_count.argtypes = [C.c_void_p]
     lib.lt_host_register.argtypes = [C.c_void_p, C.c_uint64]
     lib.lt_host_unregister.argtypes = [C.c_void_p]
@@ -204,6 +206,21 @@ class Context:
         if rc != 0:
             raise LtError("lt_ctx_create failed (%d): %s" % (rc, self.lib.lt_last_error(None).decode()))
         self.h = h
+        self.shared_device = None
+
+    @classmethod
+    def shared(cls, device, members):
+        """Test hook (lt_debug_ctx_create_shared): a multi-device Context of `members` members that all render on
+        `device`; shared_device is then that ordinal (None on every other Context)."""
+        self = cls.__new__(cls)
+        self.lib = load()
+        h = C.c_void_p()
+        rc = self.lib.lt_debug_ctx_create_shared(device, members, C.byref(h))
+        if rc != 0:
+            raise LtError("lt_debug_ctx_create_shared failed (%d): %s" % (rc, self.lib.lt_last_error(None).decode()))
+        self.h = h
+        self.shared_device = device
+        return self
 
     def device_count(self):
         return self.lib.lt_ctx_device_count(self.h)

@@ -18,6 +18,7 @@
 #include "lt_device.cuh"
 
 #include <cub/device/device_scan.cuh>
+#include <mutex>
 
 // LIST: thread i renders pixel M.list[i] (a masked launch); M2: and keeps the Welford sums at M.m2 (running mean only)
 template <bool STATS, bool LIST, bool M2>
@@ -556,13 +557,8 @@ int lt_launch_reflatten(const RefNode* dNodes, int nodeCount, const RefPrim* dPr
 
 // The culled mode on a tree deeper than 40 levels asks for up to (2 * 64 + 16) * 512 = 73 728 bytes.
 static const int kMaxTraversalSmem = (int)lt_traversal_smem(64, LT_BLOCK, true);
-void lt_opt_in_traversal_smem(size_t smem) {
-  if (smem <= 48 * 1024) return;
-  static bool done[64] = {};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev < 0 || dev >= 64 || done[dev]) return;
-  done[dev] = true;
+// the traversal kernels' dynamic shared-memory limit raised to kMaxTraversalSmem on the current device
+static void opt_in_traversal_kernels() {
   const void* const mine[] = {(const void*)k_flat<false, false, false>, (const void*)k_flat<true, false, false>,
                               (const void*)k_flat<false, true, false>,  (const void*)k_flat<true, true, false>,
                               (const void*)k_flat<false, true, true>,   (const void*)k_flat<true, true, true>,
@@ -573,6 +569,18 @@ void lt_opt_in_traversal_smem(size_t smem) {
   for (const void* k : mine) cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxTraversalSmem);
   for (const void* k : lt_wf_traversal_kernels)
     cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxTraversalSmem);
+}
+
+// Once per device.  A thread that finds the device done may launch at once, so call_once returns to no thread before
+// every attribute is set: several host threads render on one device when a caller drives two contexts there, and in
+// the members of a shared group (lt_debug_ctx_create_shared).
+void lt_opt_in_traversal_smem(size_t smem) {
+  if (smem <= 48 * 1024) return;
+  static std::once_flag done[64];
+  int dev = 0;
+  cudaGetDevice(&dev);
+  if (dev < 0 || dev >= 64) return;
+  std::call_once(done[dev], opt_in_traversal_kernels);
 }
 
 template <bool LIST, bool M2>

@@ -109,11 +109,44 @@ struct LtGroup {
   std::vector<cudaEvent_t> rendered, summed;
   int lastSplit = -1;               // split of the accumulators the devices hold (a change resets them)
   long long lastFloats = -1;
+  bool sharesDevice = false;        // a device ordinal is listed more than once (lt_debug_ctx_create_shared)
 };
 
 extern "C" int lt_ctx_device_count(const lt_ctx* ctx) {
   if (!ctx) return 0;
   return ctx->group ? (int)ctx->group->ctx.size() : 1;
+}
+
+// The group context over `count` member contexts, member k on device ordinals[k].  An ordinal may repeat (shared
+// groups, lt_debug_ctx_create_shared): every member is an ordinary single-GPU context with its own stream, buffers and
+// host thread either way.
+static int create_group(const int* ordinals, int count, lt_ctx** out_ctx) {
+  LtGroup* g = new LtGroup();
+  for (int a = 0; a < count; a++)
+    for (int b = a + 1; b < count; b++) g->sharesDevice |= ordinals[a] == ordinals[b];
+  for (int k = 0; k < count; k++) {
+    lt_ctx* c = nullptr;
+    int rc = lt_ctx_create(ordinals[k], &c);
+    if (rc != LT_OK) {
+      for (lt_ctx* d : g->ctx) lt_ctx_destroy(d);
+      delete g;
+      return rc;  // message already set by lt_ctx_create
+    }
+    g->ctx.push_back(c);
+  }
+  g->rendered.resize(count, nullptr);
+  g->summed.resize(count, nullptr);
+  for (int k = 0; k < count; k++) {
+    cudaSetDevice(g->ctx[k]->device);
+    cudaEventCreateWithFlags(&g->rendered[k], cudaEventDisableTiming);
+    cudaEventCreateWithFlags(&g->summed[k], cudaEventDisableTiming);
+  }
+  lt_ctx* ctx = new lt_ctx();
+  ctx->device = ordinals[0];
+  ctx->group = g;
+  ctx->stats.sm_count = g->ctx[0]->stats.sm_count;
+  *out_ctx = ctx;
+  return LT_OK;
 }
 
 extern "C" int lt_ctx_create_multi(const int* device_ordinals, int device_count, lt_ctx** out_ctx) {
@@ -126,30 +159,16 @@ extern "C" int lt_ctx_create_multi(const int* device_ordinals, int device_count,
       if (device_ordinals[a] == device_ordinals[b])
         return lt_internal_fail(nullptr, LT_ERR_INVALID, "lt_ctx_create_multi: a device ordinal is listed twice");
   if (device_count == 1) return lt_ctx_create(device_ordinals[0], out_ctx);
-  LtGroup* g = new LtGroup();
-  for (int k = 0; k < device_count; k++) {
-    lt_ctx* c = nullptr;
-    int rc = lt_ctx_create(device_ordinals[k], &c);
-    if (rc != LT_OK) {
-      for (lt_ctx* d : g->ctx) lt_ctx_destroy(d);
-      delete g;
-      return rc;  // message already set by lt_ctx_create
-    }
-    g->ctx.push_back(c);
-  }
-  g->rendered.resize(device_count, nullptr);
-  g->summed.resize(device_count, nullptr);
-  for (int k = 0; k < device_count; k++) {
-    cudaSetDevice(g->ctx[k]->device);
-    cudaEventCreateWithFlags(&g->rendered[k], cudaEventDisableTiming);
-    cudaEventCreateWithFlags(&g->summed[k], cudaEventDisableTiming);
-  }
-  lt_ctx* ctx = new lt_ctx();
-  ctx->device = device_ordinals[0];
-  ctx->group = g;
-  ctx->stats.sm_count = g->ctx[0]->stats.sm_count;
-  *out_ctx = ctx;
-  return LT_OK;
+  return create_group(device_ordinals, device_count, out_ctx);
+}
+
+extern "C" int lt_debug_ctx_create_shared(int device_ordinal, int members, lt_ctx** out_ctx) {
+  if (!out_ctx) return lt_internal_fail(nullptr, LT_ERR_INVALID, "lt_debug_ctx_create_shared: out_ctx is NULL");
+  *out_ctx = nullptr;
+  if (members < 2 || members > LT_MAX_DEVICES)
+    return lt_internal_fail(nullptr, LT_ERR_INVALID, "lt_debug_ctx_create_shared: needs 2..16 members");
+  const std::vector<int> ordinals(members, device_ordinal);
+  return create_group(ordinals.data(), members, out_ctx);
 }
 
 void lt_multi_destroy(lt_ctx* ctx) {
@@ -283,6 +302,10 @@ const std::vector<LtPlugin*>& lt_multi_plugins(const lt_ctx* ctx) { return ctx->
 static bool ensure_nccl(LtGroup* g, std::string* why) {
   if (g->ncclTried) return g->ncclReady;
   g->ncclTried = true;
+  if (g->sharesDevice) {  // NCCL gives each rank a device of its own
+    *why = "a device is listed more than once";
+    return false;
+  }
   if (!load_nccl()) {
     *why = g_nccl.why;
     return false;
@@ -307,7 +330,8 @@ static bool ensure_peers(LtGroup* g, size_t floats, std::string* why) {
     for (size_t a = 0; a < g->ctx.size() && g->peersReady; a++) {
       cudaSetDevice(g->ctx[a]->device);
       for (size_t b = 0; b < g->ctx.size(); b++) {
-        if (a == b) continue;
+        // a device reads its own memory without peer mapping (members of a shared group)
+        if (g->ctx[a]->device == g->ctx[b]->device) continue;
         int can = 0;
         cudaDeviceCanAccessPeer(&can, g->ctx[a]->device, g->ctx[b]->device);
         if (!can) {

@@ -412,9 +412,6 @@ def test_cpp_renderers_equal_the_host_form():
 
 
 def test_multi_gpu_equals_one_gpu():
-    if torch.cuda.device_count() < 2:
-        pytest.skip("needs two GPUs")
-    devices = list(range(min(torch.cuda.device_count(), 8)))
     sb = util.scene("cornell_box_lens")
     w, h = 320, 203
     p = params(L.KERNEL_GI, w, h, 4)
@@ -422,8 +419,9 @@ def test_multi_gpu_equals_one_gpu():
         sc = one.upload(sb)
         want, want_n, want_res = one.render_adaptive(sc, cam(0), p, 0.08, round_frames=4, max_frames=16)
         sc.release()
-    for G in sorted({2, len(devices)}):
-        with capi.Context(devices[:G]) as multi:
+    sizes = sorted({2, min(torch.cuda.device_count(), 8)}) if torch.cuda.device_count() >= 2 else util.group_sizes()
+    for G in sizes:
+        with util.device_group(G) as multi:
             sc = multi.upload(sb)
             for split in (L.SPLIT_AUTO, L.SPLIT_TILES):
                 p.split_mode = split

@@ -1,7 +1,7 @@
 """lt_last_stats after a call: every field describes that call and reads 0 for what the call did not measure -- the
 counters without LT_FLAG_STATS, the kernel time of an asynchronous call.  On a multi-GPU context, a device with no
 share in a call adds nothing to the call's statistics, and a call refused for its parameters leaves the devices'
-accumulators as they were.  The multi-GPU cases need two or more devices and are skipped otherwise."""
+accumulators as they were.  The multi-GPU cases run on shared groups (util.device_group) on a machine with one GPU."""
 import os
 
 import numpy as np
@@ -13,14 +13,6 @@ from lens_trace_b200 import capi, host, layouts as L
 pytestmark = pytest.mark.gpu
 
 GI_FILE = "examples/global_illumination/resources/kernels/global_illumination.cl"
-
-
-def device_count():
-    import torch
-    return torch.cuda.device_count()
-
-
-needs_two = pytest.mark.skipif("device_count() < 2", reason="needs two or more GPUs")
 
 
 def rel_diff(a, b):
@@ -76,9 +68,12 @@ def test_kernel_time_of_an_asynchronous_call():
         sc.release()
 
 
-@needs_two
 def test_devices_without_a_share_add_nothing():
-    n = min(device_count(), 8)
+    for n in util.group_sizes():
+        devices_without_a_share_add_nothing(n)
+
+
+def devices_without_a_share_add_nothing(n):
     cam = util.default_camera()
 
     def samples(frames):
@@ -90,7 +85,7 @@ def test_devices_without_a_share_add_nothing():
 
     for params, busy in ((samples, 8), (tiles, 64)):
         idle = 1 if params is samples else 8
-        with capi.Context(list(range(n))) as many:
+        with util.device_group(n) as many:
             sm = many.upload(util.scene("cornell_box"))
             many.render(sm, cam, params(idle), want_output=False)
             fresh = many.stats().kernel_launches
@@ -103,12 +98,16 @@ def test_devices_without_a_share_add_nothing():
             sm.release()
 
 
-@needs_two
 @pytest.mark.parametrize("exchange", ["nccl", "p2p"])
 def test_refused_call_leaves_the_accumulators(exchange, monkeypatch):
     """A (frames 0-3), the refused B (max_ray_depth 300), C (frames 4-7): C as after A alone."""
+    util.skip_nccl_without_two_gpus(exchange)
     monkeypatch.setenv("LT_MULTI_EXCHANGE", exchange)
-    n = min(device_count(), 8)
+    for n in util.group_sizes():
+        refused_call_leaves_the_accumulators(exchange, n)
+
+
+def refused_call_leaves_the_accumulators(exchange, n):
     sb = util.scene("cornell_box")
     w, h = 160, 96
 
@@ -123,7 +122,7 @@ def test_refused_call_leaves_the_accumulators(exchange, monkeypatch):
         s1.release()
     got = []
     for refuse in (False, True):
-        with capi.Context(list(range(n))) as many:
+        with util.device_group(n) as many:
             sm = many.upload(sb)
             many.render(sm, util.default_camera(0.0, 0), p(), want_output=False)
             if refuse:

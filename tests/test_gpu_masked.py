@@ -347,10 +347,7 @@ def test_images_above_int_max_pixels_are_refused(ctx, scenes):
 
 
 def test_multi_gpu_context_is_unsupported():
-    n = torch.cuda.device_count()
-    if n < 2:
-        pytest.skip("needs two or more devices")
-    with capi.Context(list(range(n))) as multi:
+    with util.device_group(max(2, min(torch.cuda.device_count(), 8))) as multi:
         sc = multi.upload(util.scene("cornell_box"))
         start = np.full((H, W, 3), 5.0, np.float32)
         out = dev(start)

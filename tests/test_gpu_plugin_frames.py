@@ -30,9 +30,6 @@ def device_count():
     return torch.cuda.device_count()
 
 
-needs_two = pytest.mark.skipif("device_count() < 2", reason="needs two or more GPUs")
-
-
 def rel_diff(a, b):
     return float((np.abs(a.astype(np.float64) - b) / np.maximum(np.abs(b), 1e-3)).max())
 
@@ -238,14 +235,18 @@ def test_argument_errors(ctx):
 
 # ---------------------------------------------------------------- several GPUs
 
-@needs_two
 @pytest.mark.gpu
 @pytest.mark.parametrize("exchange", ["nccl", "p2p"])
 def test_sample_split_of_a_plugin(exchange, monkeypatch):
+    util.skip_nccl_without_two_gpus(exchange)
     monkeypatch.setenv("LT_MULTI_EXCHANGE", exchange)
-    n = min(device_count(), 8)
+    for n in util.group_sizes():
+        sample_split_of_a_plugin(exchange, n)
+
+
+def sample_split_of_a_plugin(exchange, n):
     sb = util.scene("cornell_box")
-    one, many = capi.Context(0), capi.Context(list(range(n)))
+    one, many = capi.Context(0), util.device_group(n)
     s1, sm = one.upload(sb), many.upload(sb)
     p1, pm = one.plugin_load(GI), many.plugin_load(GI)
     cam = util.default_camera(0.0, 0)

@@ -23,11 +23,6 @@ FLAGS = [0, L.FLAG_MEGAKERNEL, L.FLAG_WAVEFRONT, L.FLAG_NO_THREADED, L.FLAG_NO_S
 GI_PLUGIN = os.path.join(util.ROOT, "tests", "plugins", "gi_plugin.cu")
 
 
-def device_count():
-    import torch
-    return torch.cuda.device_count()
-
-
 def interior(prims):
     """the primitives of the objects inside the Cornell room (not its walls, floor or ceiling)"""
     lo = np.minimum(np.minimum(prims["a"], prims["b"]), prims["c"])
@@ -394,12 +389,15 @@ def test_device_form_from_a_torch_tensor(ctx):
     b.release()
 
 
-@pytest.mark.skipif("device_count() < 2", reason="needs two or more GPUs")
 def test_refit_every_device_copy():
+    for n in util.group_sizes():
+        refit_every_device_copy(n)
+
+
+def refit_every_device_copy(n):
     sb = util.scene("cornell_box")
     prims = translated(sb.prims)
-    n = min(device_count(), 8)
-    with capi.Context(0) as one, capi.Context(list(range(n))) as many:
+    with capi.Context(0) as one, util.device_group(n) as many:
         a, m = one.upload(sb), many.upload(sb)
         one.refit(a, prims)
         many.refit(m, prims)

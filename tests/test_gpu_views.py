@@ -237,21 +237,19 @@ def test_cpp_renderer_views():
 
 
 def test_multi_gpu_views_equal_single_gpu():
-    import torch
-    n = torch.cuda.device_count()
-    if n < 2:
-        pytest.skip("needs two or more devices")
     cams = cameras(5)
     p = capi.make_params(L.KERNEL_GI, 101, 75, max_ray_depth=4, frames=3, accum_mode=L.ACCUM_RUNNING_MEAN)
     with capi.Context(0) as one:
         sc = one.upload(util.scene("cornell_box"))
         want = one.render_views(sc, cams, p)
         sc.release()
-    with capi.Context(list(range(n))) as multi:
-        sc = multi.upload(util.scene("cornell_box"))
-        got = multi.render_views(sc, cams, p)
-        p.split_mode = 1
-        with pytest.raises(capi.LtError):
-            multi.render_views(sc, cams, p)
-        sc.release()
-    util.assert_bit_equal(got, want, "multi-GPU views")
+    for n in util.group_sizes():
+        p.split_mode = L.SPLIT_AUTO
+        with util.device_group(n) as multi:
+            sc = multi.upload(util.scene("cornell_box"))
+            got = multi.render_views(sc, cams, p)
+            p.split_mode = 1
+            with pytest.raises(capi.LtError):
+                multi.render_views(sc, cams, p)
+            sc.release()
+        util.assert_bit_equal(got, want, "multi-GPU views, %d devices" % n)

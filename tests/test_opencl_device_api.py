@@ -250,21 +250,19 @@ def test_a_group_whose_stacks_do_not_fit_is_refused():
     c.close()
 
 
-def device_count():
-    import torch
-    return torch.cuda.device_count()
-
-
 def rel_diff(a, b):
     return float((np.abs(a.astype(np.float64) - b) / np.maximum(np.abs(b), 1e-3)).max())
 
 
-@pytest.mark.skipif("device_count() < 2", reason="needs two or more GPUs")
 @pytest.mark.gpu
 def test_sample_split_of_the_ported_file():
-    n = min(device_count(), 8)
+    for n in util.group_sizes():
+        sample_split_of_the_ported_file(n)
+
+
+def sample_split_of_the_ported_file(n):
     sb = util.scene("cornell_box")
-    one, many = capi.Context(0), capi.Context(list(range(n)))
+    one, many = capi.Context(0), util.device_group(n)
     s1, sm = one.upload(sb), many.upload(sb)
     p1, pm = one.plugin_load(GI_CL), many.plugin_load(GI_CL)
     cam = util.default_camera(0.0, 0)

@@ -417,11 +417,8 @@ def test_error_cases(ctx):
 
 @pytest.mark.gpu
 def test_multi_gpu_context_is_refused():
-    import torch
-    if torch.cuda.device_count() < 2:
-        pytest.skip("needs two GPUs")
     prims, mats, _ = _load(os.path.join(util.MODELS, "cornell_box.obj"))
-    c = capi.Context([0, 1])
+    c = util.device_group(2)
     assert _rc(c, prims, mats) == -4
     assert "single-GPU context" in c.lib.lt_last_error(c.h).decode()
     c.close()

@@ -3,7 +3,7 @@ import os
 
 import numpy as np
 
-from lens_trace_b200 import host, layouts as L
+from lens_trace_b200 import capi, host, layouts as L
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 MODELS = os.path.join(ROOT, "resources", "models")
@@ -22,6 +22,38 @@ def scene(name):
 def default_camera(yaw=0.0, frame_count=0):
     # the camera every reference test and example uses (tests/cuda_renderer_test.cc:19)
     return L.make_camera(0, 2.5, -50, yaw, frame_count)
+
+
+def device_group(n):
+    """A multi-device Context of n members: devices 0 .. n-1 when torch sees that many, otherwise a shared group of n
+    members on device 0 (capi.Context.shared), which runs every line of the multi-GPU code except the NCCL and peer
+    mapping transport.  Use it in a `with` block, so that no member context or thread outlives the test."""
+    import torch
+    if torch.cuda.device_count() >= n:
+        return capi.Context(list(range(n)))
+    return capi.Context.shared(0, n)
+
+
+def is_shared(ctx):
+    """Whether a Context from device_group is a shared group (every member on one device)."""
+    return ctx.shared_device is not None
+
+
+def skip_nccl_without_two_gpus(exchange):
+    """A test of the NCCL exchange needs a real group: a shared group's sample split always runs the p2p kernel, so on
+    one GPU the nccl case would test that path a second time."""
+    import pytest
+    import torch
+    if exchange == "nccl" and torch.cuda.device_count() < 2:
+        pytest.skip("the nccl exchange needs two or more GPUs (a shared group combines with the p2p kernel)")
+
+
+def group_sizes():
+    """The member counts the multi-device tests use: every real device (up to 8) when there are two or more, and on
+    one GPU 3 (not a power of two) and 8 (the largest count of a real group)."""
+    import torch
+    n = torch.cuda.device_count()
+    return [min(n, 8)] if n >= 2 else [3, 8]
 
 
 def bits(a):
