@@ -411,8 +411,8 @@ int lt_debug_traversal_tree(const void* nodes, uint64_t node_bytes, int32_t prim
 /* Test hook: 1 when the pruned threaded copies of an uploaded scene are a traversal tree, 0 when not (also for
  * scenes without host-built copies), < 0 on error. */
 int lt_debug_scene_traversal_tree(const lt_scene* scene);
-/* Test hook: the bytes of device memory a scene holds (all devices' copies of a multi-GPU scene), counted at each
- * allocation and release the library makes for it. */
+/* Test hook: the bytes of device memory a scene holds (all devices' copies of a multi-GPU scene): the sum of the
+ * buffers it holds at the time of the call. */
 int lt_debug_scene_bytes(const lt_scene* scene, uint64_t* out_bytes);
 
 /* Test hook: full != 0 makes launches on `scene` (single-GPU) walk the full threaded copies for every ray, 0 restores

@@ -109,33 +109,6 @@ int lt_internal_fail(lt_ctx* ctx, int code, const std::string& msg) { return fai
 
 int lt_internal_ctx_device(const lt_ctx* ctx) { return ctx->device; }
 
-// cudaMalloc / cudaFree of a buffer the scene owns, counted in s->deviceBytes (lt_debug_scene_bytes)
-template <class T>
-static cudaError_t scene_alloc(lt_scene* s, T** p, size_t bytes) {
-  const cudaError_t e = cudaMalloc((void**)p, bytes);
-  if (e == cudaSuccess) s->deviceBytes += bytes;
-  return e;
-}
-template <class T>
-static void scene_free(lt_scene* s, T** p, size_t bytes) {
-  if (*p) s->deviceBytes -= bytes;
-  cudaFree(*p);
-  *p = nullptr;
-}
-
-// A grow-only buffer of the context: *p holds at least `want` units of `unit` bytes, *have counts them.  A new
-// allocation keeps nothing of the old contents, and *have stays 0 when it fails.
-template <class T, class N>
-static cudaError_t ctx_grow(T** p, N* have, N want, size_t unit) {
-  if (*have >= want) return cudaSuccess;
-  if (*p) cudaFree(*p);
-  *p = nullptr;
-  *have = 0;
-  const cudaError_t e = cudaMalloc((void**)p, (size_t)want * unit);
-  if (e == cudaSuccess) *have = want;
-  return e;
-}
-
 // Host primitives of an upload, a device build or a refit: every material index in [0, matCount) and, with `finite`,
 // every vertex coordinate finite.  `w` starts the error message.
 static int check_prims(lt_ctx* ctx, const RefPrim* prims, uint64_t n, uint64_t matCount, bool finite,
@@ -178,66 +151,43 @@ extern "C" int lt_ctx_create(int device_ordinal, lt_ctx** out_ctx) {
   ctx->device = device_ordinal;
   ctx->stats.sm_count = prop.multiProcessorCount;
   ctx->totalMem = prop.totalGlobalMem;
-  cudaError_t e2 = cudaStreamCreateWithFlags(&ctx->ownStream, cudaStreamNonBlocking);
-  if (e2 == cudaSuccess) e2 = cudaEventCreate(&ctx->ev0);
-  if (e2 == cudaSuccess) e2 = cudaEventCreate(&ctx->ev1);
-  if (e2 == cudaSuccess) e2 = cudaMalloc(&ctx->dCounters, sizeof(LtCounters));
-  if (e2 == cudaSuccess) e2 = cudaMalloc(&ctx->dWork, 256);
-  if (e2 == cudaSuccess) e2 = cudaStreamCreateWithFlags(&ctx->wfAux.extra, cudaStreamNonBlocking);
-  if (e2 == cudaSuccess) e2 = cudaEventCreateWithFlags(&ctx->wfAux.fork, cudaEventDisableTiming);
-  for (int k = 0; k < 2; k++)
-    if (e2 == cudaSuccess) e2 = cudaEventCreateWithFlags(&ctx->wfAux.order[k], cudaEventDisableTiming);
+  cudaError_t e2 = ctx->ownStream.create();
+  ctx->stream = ctx->ownStream.get();
+  if (e2 == cudaSuccess) e2 = ctx->ev.grow(2, cudaEventDefault);
+  if (e2 == cudaSuccess) e2 = ctx->dCounters.grow(1);
+  if (e2 == cudaSuccess) e2 = ctx->dWork.grow(64);  // 256 bytes
+  if (e2 == cudaSuccess) e2 = ctx->wfExtra.create();
+  if (e2 == cudaSuccess) e2 = ctx->wfEvents.grow(3, cudaEventDisableTiming);
   if (e2 != cudaSuccess) {
     std::string m = std::string("lt_ctx_create: ") + cudaGetErrorString(e2);
     delete ctx;
     return fail(nullptr, LT_ERR_CUDA, m);
   }
-  ctx->stream = ctx->ownStream;
   *out_ctx = ctx;
   return LT_OK;
 }
 
+lt_ctx::lt_ctx() = default;
+
+// A single-GPU context waits for its streams (the caller's one included) before its members release what they hold.
+// A group context has no stream of its own and touches no device: lt_multi_destroy has released its members.
+lt_ctx::~lt_ctx() {
+  if (!ownStream.get()) return;
+  cudaSetDevice(device);
+  cudaStreamSynchronize(stream);
+  if (wfExtra.get()) cudaStreamSynchronize(wfExtra.get());
+  for (LtPlugin* p : plugins) lt_plugin_free(p);
+}
+
 extern "C" void lt_ctx_destroy(lt_ctx* ctx) {
-  if (!ctx) return;
-  if (ctx->group) {
-    lt_multi_destroy(ctx);
-    delete ctx;
-    return;
-  }
-  cudaSetDevice(ctx->device);
-  cudaStreamSynchronize(ctx->stream);
-  if (ctx->dOut) cudaFree(ctx->dOut);
-  if (ctx->dCounters) cudaFree(ctx->dCounters);
-  if (ctx->dWork) cudaFree(ctx->dWork);
-  if (ctx->wfWorkspace) cudaFree(ctx->wfWorkspace);
-  if (ctx->dCamera) cudaFree(ctx->dCamera);
-  if (ctx->dSample) cudaFree(ctx->dSample);
-  if (ctx->dViews) cudaFree(ctx->dViews);
-  if (ctx->dViewFrameCounts) cudaFree(ctx->dViewFrameCounts);
-  if (ctx->dMaskList) cudaFree(ctx->dMaskList);
-  if (ctx->dAdaptive) cudaFree(ctx->dAdaptive);
-  delete ctx->copyPool;
-  if (ctx->stage) cudaFreeHost(ctx->stage);
-  for (cudaEvent_t e : ctx->stageEvents) cudaEventDestroy(e);
-  for (LtPlugin* p : ctx->plugins) lt_plugin_free(p);
-  for (cudaEvent_t e : ctx->traceEvents) cudaEventDestroy(e);
-  if (ctx->ev0) cudaEventDestroy(ctx->ev0);
-  if (ctx->ev1) cudaEventDestroy(ctx->ev1);
-  if (ctx->wfAux.extra) {
-    cudaStreamSynchronize(ctx->wfAux.extra);
-    cudaStreamDestroy(ctx->wfAux.extra);
-  }
-  if (ctx->wfAux.fork) cudaEventDestroy(ctx->wfAux.fork);
-  for (cudaEvent_t e : ctx->wfAux.order)
-    if (e) cudaEventDestroy(e);
-  if (ctx->ownStream) cudaStreamDestroy(ctx->ownStream);
+  if (ctx && ctx->group) lt_multi_destroy(ctx);
   delete ctx;
 }
 
 extern "C" int lt_ctx_set_stream(lt_ctx* ctx, void* cuda_stream) {
   if (!ctx) return fail(nullptr, LT_ERR_INVALID, "lt_ctx_set_stream: ctx is NULL");
   if (ctx->group) return fail(ctx, LT_ERR_UNSUPPORTED, "lt_ctx_set_stream: a multi-GPU context renders on its own per-device streams");
-  ctx->stream = cuda_stream ? (cudaStream_t)cuda_stream : ctx->ownStream;
+  ctx->stream = cuda_stream ? (cudaStream_t)cuda_stream : ctx->ownStream.get();
   return LT_OK;
 }
 
@@ -251,16 +201,6 @@ extern "C" void lt_scene_release(lt_ctx* ctx, lt_scene* s) {
     cudaSetDevice(ctx->device);
     cudaStreamSynchronize(ctx->stream);
   }
-  cudaFree(s->dNodes);
-  cudaFree(s->dPrims);
-  cudaFree(s->dMats);
-  cudaFree(s->dLights);
-  cudaFree(s->dWide);
-  cudaFree(s->dTris);
-  cudaFree(s->dThread);
-  cudaFree(s->dRank);
-  cudaFree(s->dThreadBig);
-  cudaFree(s->dRefit);
   delete s;
 }
 
@@ -274,7 +214,7 @@ extern "C" int lt_debug_scene_traversal_tree(const lt_scene* scene) {
 // copies, or `full`) the full copies, which are also the layout of the device-built dThreadBig.
 static void set_pruned_copies(lt_scene* s, bool full) {
   LtSceneDev& d = s->dev;
-  const bool pruned = s->dThread != nullptr && !full;
+  const bool pruned = s->dThread.get() != nullptr && !full;
   d.prunedBase = pruned ? 8 * d.nodeCount : 0;
   d.prunedStride = pruned ? s->threadStride : d.nodeCount;
 }
@@ -289,80 +229,73 @@ extern "C" int lt_debug_scene_full_threaded(lt_scene* scene, int full) {
 // 48-byte triangles (re-flatten through the inner-node ranks dInnerRank), the threaded copies the scene keeps
 // (`copies`: built on the host for small trees, the one pass that may grow dThread or add dRank, or on the device for
 // large ones), and the launch state.  Upload and refit share it, so a refitted scene is what an upload of its buffers
-// makes.  ev0 must already be recorded on the stream; records ev1 and sets upload_ms.
+// makes.  ev[0] must already be recorded on the stream; records ev[1] and sets upload_ms.
 static cudaError_t derive_scene(lt_ctx* ctx, lt_scene* s, const int* dInnerRank, LtTree copies, const RefNode& root) {
   LtSceneDev& d = s->dev;
   const int nNodes = d.nodeCount, nPrims = d.primCount;
   cudaError_t e = cudaSuccess;
   auto A = [&](cudaError_t r) { if (e == cudaSuccess) e = r; };
   cudaStream_t st = ctx->stream;
-  lt_launch_reflatten(s->dNodes, nNodes, s->dPrims, nPrims, dInnerRank, s->dWide, s->dTris, st);
+  lt_launch_reflatten(s->dNodes.get(), nNodes, s->dPrims.get(), nPrims, dInnerRank, s->dWide.get(), s->dTris.get(), st);
   A(cudaGetLastError());
   std::vector<int> hRank;
   if (e == cudaSuccess && copies == LT_TREE_HOST_THREADED) {
     std::vector<RefNode> hNodes((size_t)nNodes);
     std::vector<LtThreadNode> hThread;
-    A(cudaMemcpyAsync(hNodes.data(), s->dNodes, sizeof(RefNode) * (size_t)nNodes, cudaMemcpyDeviceToHost, st));
+    A(cudaMemcpyAsync(hNodes.data(), s->dNodes.get(), sizeof(RefNode) * (size_t)nNodes, cudaMemcpyDeviceToHost, st));
     A(cudaStreamSynchronize(st));
     if (e == cudaSuccess) {
       s->threadStride = lt_build_threaded(hNodes.data(), nNodes, nPrims, hThread, hRank);
-      if (hThread.size() > s->threadRecords) {  // the pruned copies' size follows the boxes
-        scene_free(s, &s->dThread, sizeof(LtThreadNode) * s->threadRecords);
-        s->threadRecords = 0;
-        A(scene_alloc(s, &s->dThread, sizeof(LtThreadNode) * hThread.size()));
-        if (e == cudaSuccess) s->threadRecords = hThread.size();
-      }
-      A(cudaMemcpyAsync(s->dThread, hThread.data(), sizeof(LtThreadNode) * hThread.size(), cudaMemcpyHostToDevice, st));
+      A(s->dThread.grow(hThread.size()));  // the pruned copies' size follows the boxes
+      A(cudaMemcpyAsync(s->dThread.get(), hThread.data(), sizeof(LtThreadNode) * hThread.size(), cudaMemcpyHostToDevice,
+                        st));
       if (!hRank.empty()) {
-        if (!s->dRank) A(scene_alloc(s, &s->dRank, sizeof(int) * hRank.size()));
-        A(cudaMemcpyAsync(s->dRank, hRank.data(), sizeof(int) * hRank.size(), cudaMemcpyHostToDevice, st));
+        A(s->dRank.grow(hRank.size()));
+        A(cudaMemcpyAsync(s->dRank.get(), hRank.data(), sizeof(int) * hRank.size(), cudaMemcpyHostToDevice, st));
       }
       A(cudaStreamSynchronize(st));  // hThread and hRank are pageable and go out of scope
     }
   }
   // large trees: the threaded copies are built on the device and used by coherent-ray launches only (plan_tree)
   if (e == cudaSuccess && copies == LT_TREE_DEVICE_THREADED) {
-    if (!s->dThreadBig && scene_alloc(s, &s->dThreadBig, sizeof(LtThreadNode) * 8 * (size_t)nNodes) != cudaSuccess) {
+    if (s->dThreadBig.grow(8 * (size_t)nNodes) != cudaSuccess)
       cudaGetLastError();  // no memory for the copies: the stack traversal serves every launch
-      s->dThreadBig = nullptr;
-    }
-    if (s->dThreadBig) {
-      lt_launch_build_threaded(s->dNodes, nNodes, s->dThreadBig, st);
+    if (s->dThreadBig.get()) {
+      lt_launch_build_threaded(s->dNodes.get(), nNodes, s->dThreadBig.get(), st);
       A(cudaGetLastError());
     }
   }
-  A(cudaEventRecord(ctx->ev1, st));
+  A(cudaEventRecord(ctx->ev[1], st));
   A(cudaStreamSynchronize(st));
   if (e != cudaSuccess) return e;
-  cudaEventElapsedTime(&ctx->stats.upload_ms, ctx->ev0, ctx->ev1);
-  d.wnodes = s->dWide;
-  d.tris = s->dTris;
+  cudaEventElapsedTime(&ctx->stats.upload_ms, ctx->ev[0], ctx->ev[1]);
+  d.wnodes = s->dWide.get();
+  d.tris = s->dTris.get();
   for (int k = 0; k < 3; k++) {
     d.rootMin[k] = root.boundsMin[k];
     d.rootMax[k] = root.boundsMax[k];
   }
   d.rootRef = root.primitiveCount > 0 ? ~root.offset : 0;  // inner root is wide node 0
   d.rootCount = root.primitiveCount;
-  d.tnodes = s->dThread;
-  d.rank = hRank.empty() ? nullptr : s->dRank;
+  d.tnodes = s->dThread.get();
+  d.rank = hRank.empty() ? nullptr : s->dRank.get();
   set_pruned_copies(s, false);
   return cudaSuccess;
 }
 
-// Allocates the re-flattened buffers, derives them (derive_scene) and fills the device-side scene descriptor.  ev0
+// Allocates the re-flattened buffers, derives them (derive_scene) and fills the device-side scene descriptor.  ev[0]
 // must already be recorded on the stream; on failure the scene is released.
 static int finish_scene(lt_ctx* ctx, lt_scene* s, int nNodes, int nPrims, int nMats, const RefNode& root,
                         int stackDepth, const char* who) {
-  int* dFlags = nullptr;
-  int* dRank = nullptr;
-  void* dTemp = nullptr;
+  LtBuf<int> flags, rank;
+  LtBuf<char> temp;
   int nInner = (nNodes - 1) / 2;  // a full binary tree with one primitive slot per leaf
   if (nNodes == 1) nInner = 0;
   size_t tempBytes = lt_scan_temp_bytes(nNodes);
   LtSceneDev& d = s->dev;
-  d.prims = s->dPrims;
-  d.mats = s->dMats;
-  d.lights = s->dLights;
+  d.prims = s->dPrims.get();
+  d.mats = s->dMats.get();
+  d.lights = s->dLights.get();
   d.stackDepth = stackDepth;
   d.nodeCount = nNodes;
   d.primCount = nPrims;
@@ -370,21 +303,19 @@ static int finish_scene(lt_ctx* ctx, lt_scene* s, int nNodes, int nPrims, int nM
   cudaError_t e = cudaSuccess;
   auto A = [&](cudaError_t r) { if (e == cudaSuccess) e = r; };
   cudaStream_t st = ctx->stream;
-  A(scene_alloc(s, &s->dWide, sizeof(LtWideNode) * (size_t)(nInner > 0 ? nInner : 1)));
-  A(scene_alloc(s, &s->dTris, sizeof(LtTri) * (size_t)nPrims));
-  A(cudaMalloc(&dFlags, sizeof(int) * (size_t)nNodes));
-  A(cudaMalloc(&dRank, sizeof(int) * (size_t)nNodes));
-  A(cudaMalloc(&dTemp, tempBytes ? tempBytes : 16));
+  A(s->dWide.grow(nInner > 0 ? nInner : 1));
+  A(s->dTris.grow(nPrims));
+  A(flags.grow(nNodes));
+  A(rank.grow(nNodes));
+  A(temp.grow(tempBytes ? tempBytes : 16));
   if (e == cudaSuccess) {
-    lt_launch_inner_flags(s->dNodes, nNodes, dFlags, st);
-    lt_launch_exclusive_scan(dTemp, tempBytes, dFlags, dRank, nNodes, st);
+    lt_launch_inner_flags(s->dNodes.get(), nNodes, flags.get(), st);
+    lt_launch_exclusive_scan(temp.get(), tempBytes, flags.get(), rank.get(), nNodes, st);
     A(cudaGetLastError());
   }
-  if (e == cudaSuccess) A(derive_scene(ctx, s, dRank, lt_plan_threaded_copies(nNodes, ctx->totalMem, ctx->limits), root));
+  if (e == cudaSuccess)
+    A(derive_scene(ctx, s, rank.get(), lt_plan_threaded_copies(nNodes, ctx->totalMem, ctx->limits), root));
   cudaStreamSynchronize(st);
-  cudaFree(dFlags);
-  cudaFree(dRank);
-  cudaFree(dTemp);
   if (e != cudaSuccess) {
     lt_scene_release(ctx, s);
     return fail(ctx, LT_ERR_CUDA, std::string(who) + ": " + cudaGetErrorString(e));
@@ -413,30 +344,29 @@ static int build_scene_on_device(lt_ctx* ctx, LtBvhBuilder builder, const char* 
   CK(cudaSetDevice(ctx->device));
   int n = (int)nPrims, nNodes = 2 * n - 1;
   lt_scene* s = new lt_scene();
-  RefPrim* dInput = nullptr;
-  void* scratch = nullptr;
-  size_t scratchBytes = lt_bvh_scratch_bytes(n, builder);
   cudaError_t e = cudaSuccess;
   auto A = [&](cudaError_t r) { if (e == cudaSuccess) e = r; };
-  A(scene_alloc(s, &s->dNodes, sizeof(RefNode) * (size_t)nNodes));
-  A(scene_alloc(s, &s->dPrims, primitive_bytes));
-  A(scene_alloc(s, &s->dMats, material_bytes));
-  A(scene_alloc(s, &s->dLights, sizeof(RefLights)));
-  A(cudaMalloc(&dInput, primitive_bytes));
-  A(cudaMalloc(&scratch, scratchBytes));
-  cudaStream_t st = ctx->stream;
-  A(cudaEventRecord(ctx->ev0, st));
-  A(cudaMemcpyAsync(dInput, primitives, primitive_bytes, cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(s->dMats, materials, material_bytes, cudaMemcpyHostToDevice, st));
+  A(s->dNodes.grow(nNodes));
+  A(s->dPrims.grow(nPrims));
+  A(s->dMats.grow(nMats));
+  A(s->dLights.grow(1));
   int maxDepth = 0, launches = -1;
-  if (e == cudaSuccess)
-    launches = lt_launch_bvh_build(builder, dInput, n, s->dMats, (int)nMats, s->dNodes, s->dPrims, s->dLights, scratch,
-                                   scratchBytes, &maxDepth, st);
   RefNode root;
   memset(&root, 0, sizeof root);
-  if (e == cudaSuccess && launches >= 0) A(cudaMemcpy(&root, s->dNodes, sizeof root, cudaMemcpyDeviceToHost));
-  cudaFree(dInput);
-  cudaFree(scratch);
+  {  // the builder's input and scratch go before the re-flatten allocates
+    LtBuf<RefPrim> input;
+    LtBuf<char> scratch;
+    A(input.grow(nPrims));
+    A(scratch.grow(lt_bvh_scratch_bytes(n, builder)));
+    cudaStream_t st = ctx->stream;
+    A(cudaEventRecord(ctx->ev[0], st));
+    A(cudaMemcpyAsync(input.get(), primitives, primitive_bytes, cudaMemcpyHostToDevice, st));
+    A(cudaMemcpyAsync(s->dMats.get(), materials, material_bytes, cudaMemcpyHostToDevice, st));
+    if (e == cudaSuccess)
+      launches = lt_launch_bvh_build(builder, input.get(), n, s->dMats.get(), (int)nMats, s->dNodes.get(), s->dPrims.get(),
+                                     s->dLights.get(), scratch.get(), scratch.count(), &maxDepth, st);
+    if (e == cudaSuccess && launches >= 0) A(cudaMemcpy(&root, s->dNodes.get(), sizeof root, cudaMemcpyDeviceToHost));
+  }
   if (e != cudaSuccess || launches < 0) {
     lt_scene_release(ctx, s);
     return fail(ctx, LT_ERR_CUDA, w + (e != cudaSuccess ? cudaGetErrorString(e) : "build failed"));
@@ -471,13 +401,13 @@ extern "C" int lt_scene_download(lt_ctx* ctx, lt_scene* scene, void* nodes, uint
   CK(cudaStreamSynchronize(ctx->stream));
   if (nodes) {
     if (node_bytes != sizeof(RefNode) * (uint64_t)scene->dev.nodeCount) return fail(ctx, LT_ERR_INVALID, "lt_scene_download: node_bytes mismatch");
-    CK(cudaMemcpy(nodes, scene->dNodes, node_bytes, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(nodes, scene->dNodes.get(), node_bytes, cudaMemcpyDeviceToHost));
   }
   if (primitives) {
     if (primitive_bytes != sizeof(RefPrim) * (uint64_t)scene->dev.primCount) return fail(ctx, LT_ERR_INVALID, "lt_scene_download: primitive_bytes mismatch");
-    CK(cudaMemcpy(primitives, scene->dPrims, primitive_bytes, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(primitives, scene->dPrims.get(), primitive_bytes, cudaMemcpyDeviceToHost));
   }
-  if (light_container) CK(cudaMemcpy(light_container, scene->dLights, sizeof(RefLights), cudaMemcpyDeviceToHost));
+  if (light_container) CK(cudaMemcpy(light_container, scene->dLights.get(), sizeof(RefLights), cudaMemcpyDeviceToHost));
   return LT_OK;
 }
 
@@ -528,16 +458,16 @@ extern "C" int lt_scene_upload(lt_ctx* ctx, const void* nodes, uint64_t node_byt
   lt_scene* s = new lt_scene();
   cudaError_t e = cudaSuccess;
   auto A = [&](cudaError_t r) { if (e == cudaSuccess) e = r; };
-  A(scene_alloc(s, &s->dNodes, node_bytes));
-  A(scene_alloc(s, &s->dPrims, primitive_bytes));
-  A(scene_alloc(s, &s->dMats, material_bytes ? material_bytes : sizeof(RefMaterial)));
-  A(scene_alloc(s, &s->dLights, sizeof(RefLights)));
+  A(s->dNodes.grow(nNodes));
+  A(s->dPrims.grow(nPrims));
+  A(s->dMats.grow(nMats ? nMats : 1));
+  A(s->dLights.grow(1));
   cudaStream_t st = ctx->stream;
-  A(cudaEventRecord(ctx->ev0, st));
-  A(cudaMemcpyAsync(s->dNodes, nodes, node_bytes, cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(s->dPrims, primitives, primitive_bytes, cudaMemcpyHostToDevice, st));
-  if (material_bytes) A(cudaMemcpyAsync(s->dMats, materials, material_bytes, cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(s->dLights, light_container, sizeof(RefLights), cudaMemcpyHostToDevice, st));
+  A(cudaEventRecord(ctx->ev[0], st));
+  A(cudaMemcpyAsync(s->dNodes.get(), nodes, node_bytes, cudaMemcpyHostToDevice, st));
+  A(cudaMemcpyAsync(s->dPrims.get(), primitives, primitive_bytes, cudaMemcpyHostToDevice, st));
+  if (material_bytes) A(cudaMemcpyAsync(s->dMats.get(), materials, material_bytes, cudaMemcpyHostToDevice, st));
+  A(cudaMemcpyAsync(s->dLights.get(), light_container, sizeof(RefLights), cudaMemcpyHostToDevice, st));
   if (e != cudaSuccess) {
     lt_scene_release(ctx, s);
     return fail(ctx, LT_ERR_CUDA, std::string("lt_scene_upload: ") + cudaGetErrorString(e));
@@ -559,14 +489,14 @@ static int check_params(lt_ctx* ctx, const lt_scene* scene, const void* camera28
 
 static LtSceneFacts scene_facts(const lt_scene* s) {
   return {s->dev.nodeCount, s->dev.stackDepth,
-          s->dThread ? LT_TREE_HOST_THREADED : (s->dThreadBig ? LT_TREE_DEVICE_THREADED : LT_TREE_CHILD_PAIR)};
+          s->dThread.get() ? LT_TREE_HOST_THREADED : (s->dThreadBig.get() ? LT_TREE_DEVICE_THREADED : LT_TREE_CHILD_PAIR)};
 }
 
 // the scene as the plan's kernels see it: tnodes = the plan's threaded copies, NULL for the stack traversal
 static LtSceneDev scene_for_plan(const lt_scene* s, const LtPlan& plan) {
   LtSceneDev d = s->dev;
-  d.tnodes = plan.tree == LT_TREE_HOST_THREADED ? s->dThread
-             : plan.tree == LT_TREE_DEVICE_THREADED ? s->dThreadBig : nullptr;
+  d.tnodes = plan.tree == LT_TREE_HOST_THREADED ? s->dThread.get()
+             : plan.tree == LT_TREE_DEVICE_THREADED ? s->dThreadBig.get() : nullptr;
   return d;
 }
 
@@ -598,7 +528,7 @@ static int refit_scene(lt_ctx* ctx, lt_scene* s, const void* src, bool onDevice,
   // all of them, so every leaf's range must lie in the primitive buffer.
   if (s->refitLeaves == 0) {
     std::vector<RefNode> hNodes((size_t)n);
-    CK(cudaMemcpyAsync(hNodes.data(), s->dNodes, sizeof(RefNode) * (size_t)n, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(hNodes.data(), s->dNodes.get(), sizeof(RefNode) * (size_t)n, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     s->refitLeaves = 1;
     for (const RefNode& r : hNodes)
@@ -606,8 +536,8 @@ static int refit_scene(lt_ctx* ctx, lt_scene* s, const void* src, bool onDevice,
   }
   if (s->refitLeaves < 0)
     return fail(ctx, LT_ERR_INVALID, w + "a leaf's primitives run past the primitive buffer: the scene cannot be refitted");
-  if (!s->dRefit) CK(scene_alloc(s, &s->dRefit, sizeof(int) * (3 * (size_t)n + 1)));
-  int *parent = s->dRefit, *flags = parent + n, *rank = flags + n, *bad = rank + n;
+  CK(s->dRefit.grow(3 * (size_t)n + 1));
+  int *parent = s->dRefit.get(), *flags = parent + n, *rank = flags + n, *bad = rank + n;
   if (onDevice) {
     lt_launch_check_prims((const RefPrim*)src, nPrims, s->dev.matCount, bad, st);
     int why = 0;
@@ -619,33 +549,28 @@ static int refit_scene(lt_ctx* ctx, lt_scene* s, const void* src, bool onDevice,
   if (!s->refitDerived) {  // the inner-node ranks as the upload computes them, with the arrival flags as the scan's input
     // Host-built copies: room for the largest pruned copies (8 n records besides the full ones) and for the tie-break
     // table, so that no later refit allocates whatever the boxes do to the traversal tree.
-    if (s->dThread && s->threadRecords < 16 * (size_t)n) {
+    if (s->dThread.get() && s->dThread.count() < 16 * (size_t)n) {
       CK(cudaStreamSynchronize(st));
-      scene_free(s, &s->dThread, sizeof(LtThreadNode) * s->threadRecords);
-      s->threadRecords = 0;
       s->dev.tnodes = nullptr;
-      CK(scene_alloc(s, &s->dThread, sizeof(LtThreadNode) * 16 * (size_t)n));
-      s->threadRecords = 16 * (size_t)n;
+      CK(s->dThread.grow(16 * (size_t)n));
     }
-    if (s->dThread && !s->dRank) CK(scene_alloc(s, &s->dRank, sizeof(int) * 8 * (size_t)nPrims));
-    void* dTemp = nullptr;
+    if (s->dThread.get()) CK(s->dRank.grow(8 * (size_t)nPrims));
+    LtBuf<char> temp;
     const size_t tempBytes = lt_scan_temp_bytes(n);
-    CK(cudaMalloc(&dTemp, tempBytes ? tempBytes : 16));
-    lt_launch_refit_parents(s->dNodes, n, parent, st);
-    lt_launch_inner_flags(s->dNodes, n, flags, st);
-    lt_launch_exclusive_scan(dTemp, tempBytes, flags, rank, n, st);
-    const cudaError_t e = cudaStreamSynchronize(st);
-    cudaFree(dTemp);
-    CK(e);
+    CK(temp.grow(tempBytes ? tempBytes : 16));
+    lt_launch_refit_parents(s->dNodes.get(), n, parent, st);
+    lt_launch_inner_flags(s->dNodes.get(), n, flags, st);
+    lt_launch_exclusive_scan(temp.get(), tempBytes, flags, rank, n, st);
+    CK(cudaStreamSynchronize(st));
     s->refitDerived = true;
   }
-  CK(cudaEventRecord(ctx->ev0, st));
-  CK(cudaMemcpyAsync(s->dPrims, src, sizeof(RefPrim) * (size_t)nPrims,
+  CK(cudaEventRecord(ctx->ev[0], st));
+  CK(cudaMemcpyAsync(s->dPrims.get(), src, sizeof(RefPrim) * (size_t)nPrims,
                      onDevice ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, st));
-  lt_launch_refit(s->dNodes, n, s->dPrims, parent, flags, st);
+  lt_launch_refit(s->dNodes.get(), n, s->dPrims.get(), parent, flags, st);
   CK(cudaGetLastError());
   RefNode root;
-  CK(cudaMemcpyAsync(&root, s->dNodes, sizeof root, cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(&root, s->dNodes.get(), sizeof root, cudaMemcpyDeviceToHost, st));
   CK(cudaStreamSynchronize(st));  // the root box travels in the launch state
   const cudaError_t e = derive_scene(ctx, s, rank, scene_facts(s).copies, root);
   if (e != cudaSuccess) return fail(ctx, LT_ERR_CUDA, w + cudaGetErrorString(e));
@@ -685,11 +610,16 @@ extern "C" int lt_scene_refit_device(lt_ctx* ctx, lt_scene* scene, const void* d
   return refit_scene(ctx, scene, device_primitives, true, who);
 }
 
+static uint64_t scene_bytes(const lt_scene* s) {
+  uint64_t bytes = s->dNodes.bytes() + s->dPrims.bytes() + s->dMats.bytes() + s->dLights.bytes() + s->dWide.bytes() +
+                   s->dTris.bytes() + s->dThread.bytes() + s->dRank.bytes() + s->dThreadBig.bytes() + s->dRefit.bytes();
+  for (const lt_scene* p : s->parts) bytes += scene_bytes(p);
+  return bytes;
+}
+
 extern "C" int lt_debug_scene_bytes(const lt_scene* scene, uint64_t* out_bytes) {
   if (!scene || !out_bytes) return fail(nullptr, LT_ERR_INVALID, "lt_debug_scene_bytes: NULL argument");
-  uint64_t bytes = 0;
-  for (const lt_scene* p : scene->parts) bytes += p->deviceBytes;
-  *out_bytes = scene->parts.empty() ? scene->deviceBytes : bytes;
+  *out_bytes = scene_bytes(scene);
   return LT_OK;
 }
 
@@ -724,10 +654,10 @@ static void stats_add(lt_stats* sum, const lt_stats& s) {
 }
 
 int lt_internal_ensure_out(lt_ctx* ctx, size_t floats) {
-  if (ctx->outFloats >= floats) return LT_OK;
-  CK(ctx_grow(&ctx->dOut, &ctx->outFloats, floats, sizeof(float)));
-  const cudaError_t e = cudaMemsetAsync(ctx->dOut, 0, floats * sizeof(float), ctx->stream);
-  if (e != cudaSuccess) ctx->outFloats = 0;  // not zeroed: the next call allocates it anew
+  if (ctx->dOut.count() >= floats) return LT_OK;
+  CK(ctx->dOut.grow(floats));
+  const cudaError_t e = cudaMemsetAsync(ctx->dOut.get(), 0, floats * sizeof(float), ctx->stream);
+  if (e != cudaSuccess) ctx->dOut.reset();  // not zeroed: the next call allocates it anew
   CK(e);
   return LT_OK;
 }
@@ -743,9 +673,8 @@ static int render_common(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, float*
       lt_plan_render(L, scene_facts(scene), ctx->totalMem, ctx->stats.sm_count, ctx->limits, viewCount, listed);
   if (plan.error != LT_OK) return fail(ctx, plan.error, plan.message);
   const bool stats = plan.stats;
-  if (stats) CK(cudaMemsetAsync(ctx->dCounters, 0, sizeof(LtCounters), ctx->stream));
-  if (plan.pipeline == LT_PIPE_WAVEFRONT &&
-      ctx_grow(&ctx->wfWorkspace, &ctx->wfBytes, plan.workspaceBytes, 1) != cudaSuccess) {
+  if (stats) CK(cudaMemsetAsync(ctx->dCounters.get(), 0, sizeof(LtCounters), ctx->stream));
+  if (plan.pipeline == LT_PIPE_WAVEFRONT && ctx->wfWorkspace.grow(plan.workspaceBytes) != cudaSuccess) {
     cudaGetLastError();
     if (plan.forced) return fail(ctx, LT_ERR_CUDA, "lt_render: cannot allocate the wavefront workspace");
     // not a fallback to other arithmetic: the megakernel is the same path per pixel
@@ -757,10 +686,9 @@ static int render_common(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, float*
   const int kMaxTracePairs = 8192;
   int tracePairs = 0;
   bool timeTrace = wavefront && (sync || stats);
-  if (timeTrace && ctx->traceEvents.empty()) {
-    ctx->traceEvents.resize(2 * kMaxTracePairs);
+  if (timeTrace) {
+    CK(ctx->traceEvents.grow(2 * kMaxTracePairs, cudaEventDefault));
     ctx->pairKinds.resize(kMaxTracePairs);
-    for (size_t i = 0; i < ctx->traceEvents.size(); i++) cudaEventCreate(&ctx->traceEvents[i]);
   }
   // per-kernel times are only defined when one kernel runs at a time (LT_FLAG_SERIAL / stats launches)
   const bool timeKinds = timeTrace && plan.streams == 1;
@@ -771,34 +699,37 @@ static int render_common(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, float*
     std::vector<unsigned> fc(n);
     for (int v = 0; v < viewCount; v++)
       for (int f = 0; f < L.frames; f++) fc[(size_t)v * L.frames + f] = cams[v].frameCount + (unsigned)f * L.frameStride;
-    CK(ctx_grow(&ctx->dViewFrameCounts, &ctx->viewFrameCountsSize, n, sizeof(unsigned)));
+    CK(ctx->dViewFrameCounts.grow(n));
     // pageable source: staged before the call returns, so fc may go
-    CK(cudaMemcpyAsync(ctx->dViewFrameCounts, fc.data(), n * sizeof(unsigned), cudaMemcpyHostToDevice, ctx->stream));
-    views.dFrameCounts = ctx->dViewFrameCounts;
+    CK(cudaMemcpyAsync(ctx->dViewFrameCounts.get(), fc.data(), n * sizeof(unsigned), cudaMemcpyHostToDevice,
+                       ctx->stream));
+    views.dFrameCounts = ctx->dViewFrameCounts.get();
   }
-  CK(cudaEventRecord(ctx->ev0, ctx->stream));
+  CK(cudaEventRecord(ctx->ev[0], ctx->stream));
   int launches = 0;
   if (wavefront) {
-    launches = lt_launch_render_wavefront(sc, plan, L, dOut, ctx->dCounters, ctx->wfWorkspace, ctx->stats.sm_count,
-                                          ctx->stream, timeTrace ? ctx->traceEvents.data() : nullptr, kMaxTracePairs,
-                                          &tracePairs, timeKinds ? ctx->pairKinds.data() : nullptr, &ctx->wfAux,
+    const LtWfAux aux = {ctx->wfExtra.get(), ctx->wfEvents[0], {ctx->wfEvents[1], ctx->wfEvents[2]}};
+    launches = lt_launch_render_wavefront(sc, plan, L, dOut, ctx->dCounters.get(), ctx->wfWorkspace.get(),
+                                          ctx->stats.sm_count, ctx->stream,
+                                          timeTrace ? ctx->traceEvents.data() : nullptr, kMaxTracePairs, &tracePairs,
+                                          timeKinds ? ctx->pairKinds.data() : nullptr, &aux,
                                           viewCount > 1 ? &views : nullptr, list);
   } else if (viewCount > 1) {  // the megakernels: one launch per view, back to back on the stream
     for (int v = 0; v < viewCount; v++) {
       LtLaunch Lv = L;
       Lv.cam = cams[v];
-      launches += lt_launch_render(sc, plan, Lv, dOut + (size_t)v * L.width * L.height * L.depth, ctx->dCounters,
-                                   ctx->dWork, ctx->stream);
+      launches += lt_launch_render(sc, plan, Lv, dOut + (size_t)v * L.width * L.height * L.depth,
+                                   ctx->dCounters.get(), ctx->dWork.get(), ctx->stream);
     }
   } else {
-    launches = lt_launch_render(sc, plan, L, dOut, ctx->dCounters, ctx->dWork, ctx->stream, list);
+    launches = lt_launch_render(sc, plan, L, dOut, ctx->dCounters.get(), ctx->dWork.get(), ctx->stream, list);
   }
   CK(cudaGetLastError());
-  CK(cudaEventRecord(ctx->ev1, ctx->stream));
+  CK(cudaEventRecord(ctx->ev[1], ctx->stream));
   ctx->stats.kernel_launches = launches;
   if (sync || stats) {
     CK(cudaStreamSynchronize(ctx->stream));
-    CK(cudaEventElapsedTime(&ctx->stats.kernel_ms, ctx->ev0, ctx->ev1));
+    CK(cudaEventElapsedTime(&ctx->stats.kernel_ms, ctx->ev[0], ctx->ev[1]));
     if (!wavefront) {
       ctx->stats.trace_ms = ctx->stats.kernel_ms;
       ctx->stats.trace_launches = launches;
@@ -822,7 +753,7 @@ static int render_common(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, float*
   }
   if (stats) {
     LtCounters h;
-    CK(cudaMemcpy(&h, ctx->dCounters, sizeof(h), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(&h, ctx->dCounters.get(), sizeof(h), cudaMemcpyDeviceToHost));
     ctx->stats.rays = h.rays;
     ctx->stats.node_tests = h.nodeTests;
     ctx->stats.tri_tests = h.triTests;
@@ -877,9 +808,9 @@ extern "C" int lt_render_masked_device(lt_ctx* ctx, lt_scene* scene, const void*
     if (int rc = check_device_memory(ctx, device_m2, alignof(float), w, "device_m2")) return rc;
   CK(cudaSetDevice(ctx->device));
   const size_t pixels = (size_t)L.width * L.height;
-  CK(ctx_grow(&ctx->dMaskList, &ctx->maskListSize, kMaskListAt + pixels, sizeof(int)));
-  int* dCount = ctx->dMaskList;
-  int* dList = ctx->dMaskList + kMaskListAt;
+  CK(ctx->dMaskList.grow(kMaskListAt + pixels));
+  int* dCount = ctx->dMaskList.get();
+  int* dList = dCount + kMaskListAt;
   lt_launch_mask_compact(device_mask, L.width, L.height, dList, dCount, ctx->stream);
   CK(cudaGetLastError());
   // the plan sizes the launch by the listed pixels: their count comes back to the host (no mask: all of them)
@@ -902,9 +833,9 @@ static int adaptive_loop(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, const 
   CK(cudaSetDevice(ctx->device));
   *res = lt_adaptive_result{};
   const size_t pixels = (size_t)L.width * L.height, second = kMaskListAt + (pixels + kListPad - 1) / kListPad * kListPad;
-  CK(ctx_grow(&ctx->dMaskList, &ctx->maskListSize, second + pixels, sizeof(int)));
-  int* counts = ctx->dMaskList;
-  int* lists[2] = {ctx->dMaskList + kMaskListAt, ctx->dMaskList + second};
+  CK(ctx->dMaskList.grow(second + pixels));
+  int* counts = ctx->dMaskList.get();
+  int* lists[2] = {counts + kMaskListAt, counts + second};
   cudaStream_t st = ctx->stream;
   // round 1: a full image is the NULL-mask list of lt_render_masked_device, so it plans as the unmasked call
   int count = (int)pixels;
@@ -944,7 +875,7 @@ static int adaptive_loop(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, const 
     CK(cudaMemcpyAsync(&kept, &counts[1 - cur], sizeof kept, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     float ms = 0.0f;
-    CK(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+    CK(cudaEventElapsedTime(&ms, ctx->ev[0], ctx->ev[1]));
     sum.kernel_ms += ms;
     if (last) {
       res->pixels_unconverged = (uint64_t)kept;
@@ -957,7 +888,7 @@ static int adaptive_loop(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L, const 
   if (!waited && sync) {
     CK(cudaStreamSynchronize(st));
     float ms = 0.0f;
-    CK(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+    CK(cudaEventElapsedTime(&ms, ctx->ev[0], ctx->ev[1]));
     sum.kernel_ms += ms;
     waited = true;
   }
@@ -980,8 +911,8 @@ int lt_internal_render_adaptive(lt_ctx* ctx, lt_scene* scene, const LtLaunch& L,
                                 uint32_t* host_frames, int parts, int part, lt_adaptive_result* res) {
   CK(cudaSetDevice(ctx->device));
   const size_t pixels = (size_t)L.width * L.height, meanFloats = pixels * L.depth;
-  CK(ctx_grow(&ctx->dAdaptive, &ctx->adaptiveFloats, meanFloats + 4 * pixels, sizeof(float)));
-  float* dMean = ctx->dAdaptive;
+  CK(ctx->dAdaptive.grow(meanFloats + 4 * pixels));
+  float* dMean = ctx->dAdaptive.get();
   float* dM2 = dMean + meanFloats;
   unsigned* dFrames = (unsigned*)(dM2 + 3 * pixels);
   // from zero, as lt_accum_reset leaves the context accumulator
@@ -1098,39 +1029,30 @@ int lt_internal_download(lt_ctx* ctx, float* host_out, const float* dSrc, size_t
     // 4: 0.93 ms, 8: 0.76 ms per render() call
     const unsigned hw = std::thread::hardware_concurrency();
     const int threads = hw >= 16 ? 8 : (hw >= 8 ? 4 : 2);
-    ctx->copyPool = new LtCopyPool(threads - 1);
+    ctx->copyPool.reset(new LtCopyPool(threads - 1));
   }
-  if (ctx->stageBytes < (bytes < kMaxStage ? bytes : kMaxStage)) {
-    if (ctx->stage) cudaFreeHost(ctx->stage);
-    ctx->stage = nullptr;
-    ctx->stageBytes = 0;
-    size_t want = bytes < kMaxStage ? bytes : kMaxStage;
-    want = (want + kChunk - 1) / kChunk * kChunk;
-    if (cudaMallocHost(&ctx->stage, want) != cudaSuccess) {  // no pinned memory to be had: the plain copy still works
-      cudaGetLastError();
-      CK(cudaMemcpyAsync(host_out, dSrc, bytes, cudaMemcpyDeviceToHost, ctx->stream));
-      CK(cudaStreamSynchronize(ctx->stream));
-      return LT_OK;
-    }
-    ctx->stageBytes = want;
+  const size_t want = bytes < kMaxStage ? bytes : kMaxStage;
+  if (ctx->stage.count() < want && ctx->stage.grow((want + kChunk - 1) / kChunk * kChunk) != cudaSuccess) {
+    cudaGetLastError();  // no pinned memory to be had: the plain copy still works
+    CK(cudaMemcpyAsync(host_out, dSrc, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return LT_OK;
   }
+  const size_t room = ctx->stage.count();
   for (size_t done = 0; done < bytes;) {  // one pass unless the frame exceeds the staging buffer
-    const size_t pass = bytes - done < ctx->stageBytes ? bytes - done : ctx->stageBytes;
+    const size_t pass = bytes - done < room ? bytes - done : room;
     const int chunks = (int)((pass + kChunk - 1) / kChunk);
-    while ((int)ctx->stageEvents.size() < chunks) {
-      cudaEvent_t e;
-      CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-      ctx->stageEvents.push_back(e);
-    }
+    CK(ctx->stageEvents.grow(chunks, cudaEventDisableTiming));
     for (int c = 0; c < chunks; c++) {
       const size_t off = (size_t)c * kChunk, n = pass - off < kChunk ? pass - off : kChunk;
-      CK(cudaMemcpyAsync(ctx->stage + off, (const char*)dSrc + done + off, n, cudaMemcpyDeviceToHost, ctx->stream));
+      CK(cudaMemcpyAsync(ctx->stage.get() + off, (const char*)dSrc + done + off, n, cudaMemcpyDeviceToHost,
+                         ctx->stream));
       CK(cudaEventRecord(ctx->stageEvents[c], ctx->stream));
     }
     // host side: a small pool of copier threads (no CUDA calls in them); this thread waits for the chunks' DMA and
     // publishes how many have landed, then copies along
     LtCopyPool& pool = *ctx->copyPool;
-    pool.begin((char*)host_out + done, ctx->stage, pass, kChunk, chunks);
+    pool.begin((char*)host_out + done, ctx->stage.get(), pass, kChunk, chunks);
     cudaError_t err = cudaSuccess;
     for (int c = 0; c < chunks; c++) {
       cudaError_t e = cudaEventSynchronize(ctx->stageEvents[c]);
@@ -1154,9 +1076,9 @@ extern "C" int lt_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, con
   size_t floats = (size_t)L.width * L.height * L.depth;
   rc = lt_internal_ensure_out(ctx, floats);
   if (rc != LT_OK) return rc;
-  rc = render_common(ctx, scene, L, ctx->dOut, true);
+  rc = render_common(ctx, scene, L, ctx->dOut.get(), true);
   if (rc != LT_OK) return rc;
-  if (host_out) return lt_internal_download(ctx, host_out, ctx->dOut, floats * sizeof(float));
+  if (host_out) return lt_internal_download(ctx, host_out, ctx->dOut.get(), floats * sizeof(float));
   return LT_OK;
 }
 
@@ -1177,16 +1099,16 @@ int lt_internal_render_views(lt_ctx* ctx, lt_scene* scene, LtLaunch L, const Ref
   L.cam = cams[0];  // the camera of a single view
   CK(cudaSetDevice(ctx->device));
   const size_t image = (size_t)L.width * L.height * L.depth, floats = image * (size_t)count;
-  CK(ctx_grow(&ctx->dViews, &ctx->viewsFloats, floats, sizeof(float)));
+  CK(ctx->dViews.grow(floats));
   // every view accumulates from zero, as after lt_accum_reset
-  CK(cudaMemsetAsync(ctx->dViews, 0, floats * sizeof(float), ctx->stream));
-  int rc = render_common(ctx, scene, L, ctx->dViews, true, cams, count);
+  CK(cudaMemsetAsync(ctx->dViews.get(), 0, floats * sizeof(float), ctx->stream));
+  int rc = render_common(ctx, scene, L, ctx->dViews.get(), true, cams, count);
   if (rc != LT_OK || !host_out) return rc;
   if (hostStride == 1)
-    return lt_internal_download(ctx, host_out + (size_t)hostFirst * image, ctx->dViews, floats * sizeof(float));
+    return lt_internal_download(ctx, host_out + (size_t)hostFirst * image, ctx->dViews.get(), floats * sizeof(float));
   for (int k = 0; k < count && rc == LT_OK; k++)
     rc = lt_internal_download(ctx, host_out + (size_t)(hostFirst + (size_t)k * hostStride) * image,
-                              ctx->dViews + (size_t)k * image, image * sizeof(float));
+                              ctx->dViews.get() + (size_t)k * image, image * sizeof(float));
   return rc;
 }
 
@@ -1249,14 +1171,15 @@ int lt_internal_render_plugin(lt_ctx* ctx, lt_scene* scene, const RefCamera& cam
   // LT_ACCUM_NONE: every frame into the output, in order (F consecutive single-frame calls); otherwise every frame into
   // the sample buffer, folded into the accumulator after it
   const bool fold = P.accum_mode != LT_ACCUM_NONE;
-  if (fold) CK(ctx_grow(&ctx->dSample, &ctx->sampleFloats, floats, sizeof(float)));
-  float* dFrame = fold ? ctx->dSample : ctx->dOut;
-  CK(ctx_grow(&ctx->dCamera, &ctx->cameraCount, P.frames, sizeof(RefCamera)));
+  if (fold) CK(ctx->dSample.grow(floats));
+  float* dFrame = fold ? ctx->dSample.get() : ctx->dOut.get();
+  CK(ctx->dCamera.grow(P.frames));
   // frame k reads its own record, frameCount = camera.frameCount + k * frame_stride
   const uint32_t stride = P.frame_stride ? P.frame_stride : 1u;
   std::vector<RefCamera> cams((size_t)P.frames, cam);
   for (int k = 0; k < P.frames; k++) cams[k].frameCount = cam.frameCount + (uint32_t)k * stride;
-  CK(cudaMemcpyAsync(ctx->dCamera, cams.data(), sizeof(RefCamera) * cams.size(), cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(ctx->dCamera.get(), cams.data(), sizeof(RefCamera) * cams.size(), cudaMemcpyHostToDevice,
+                     ctx->stream));
   if (lt_plugin_publish_scene(plugin, &scene->dev, ctx->stream, &err) != 0)
     return fail(ctx, LT_ERR_CUDA, std::string(who) + ": " + err);
   // pixels outside every work block (the remainder of W / wbx and H / wby) read 0; the reference leaves them undefined
@@ -1267,29 +1190,30 @@ int lt_internal_render_plugin(lt_ctx* ctx, lt_scene* scene, const RefCamera& cam
   L.depth = P.depth;
   L.accumMode = P.accum_mode;
   L.accumWeight = P.accum_weight;
-  CK(cudaEventRecord(ctx->ev0, ctx->stream));
+  CK(cudaEventRecord(ctx->ev[0], ctx->stream));
   int launches = 0;
+  const lt_scene& sc = *scene;
   for (int k = 0; k < P.frames; k++) {
-    const RefCamera* dCam = ctx->dCamera + k;
-    const int n = cl ? lt_plugin_launch_cl(plugin, run.kernelMode, &scene->dev, scene->dNodes, scene->dPrims,
-                                           scene->dMats, scene->dLights, dCam, dFrame, P.width, P.height, P.depth,
+    const RefCamera* dCam = ctx->dCamera.get() + k;
+    const int n = cl ? lt_plugin_launch_cl(plugin, run.kernelMode, &sc.dev, sc.dNodes.get(), sc.dPrims.get(),
+                                           sc.dMats.get(), sc.dLights.get(), dCam, dFrame, P.width, P.height, P.depth,
                                            run.wbx, run.wby, run.bx, run.by, ctx->stream, &err)
-                     : (lt_plugin_launch(plugin, run.kernelMode, &scene->dev, scene->dNodes, scene->dPrims, scene->dMats,
-                                         scene->dLights, dCam, dFrame, P.width, P.height, P.depth, run.bx, run.by,
-                                         ctx->stream, &err) == 0 ? 1 : -1);
+                     : (lt_plugin_launch(plugin, run.kernelMode, &sc.dev, sc.dNodes.get(), sc.dPrims.get(),
+                                         sc.dMats.get(), sc.dLights.get(), dCam, dFrame, P.width, P.height, P.depth,
+                                         run.bx, run.by, ctx->stream, &err) == 0 ? 1 : -1);
     if (n < 0) return fail(ctx, LT_ERR_CUDA, std::string(who) + ": " + err);
     launches += n;
     if (fold) {
       L.cam = cams[k];
-      launches += lt_launch_plugin_accumulate(L, dFrame, ctx->dOut, ctx->stats.sm_count, ctx->stream);
+      launches += lt_launch_plugin_accumulate(L, dFrame, ctx->dOut.get(), ctx->stats.sm_count, ctx->stream);
     }
   }
   CK(cudaGetLastError());
-  CK(cudaEventRecord(ctx->ev1, ctx->stream));
+  CK(cudaEventRecord(ctx->ev[1], ctx->stream));
   ctx->stats.kernel_launches = launches;
   if (sync) {
     CK(cudaStreamSynchronize(ctx->stream));
-    CK(cudaEventElapsedTime(&ctx->stats.kernel_ms, ctx->ev0, ctx->ev1));
+    CK(cudaEventElapsedTime(&ctx->stats.kernel_ms, ctx->ev[0], ctx->ev[1]));
   }
   return LT_OK;
 }
@@ -1323,7 +1247,7 @@ static int render_plugin_once(lt_ctx* ctx, lt_scene* scene, const void* camera28
   int rc = lt_internal_render_plugin(ctx, scene, cam, P, run, true, who);
   if (rc != LT_OK) return rc;
   if (host_out)
-    return lt_internal_download(ctx, host_out, ctx->dOut, (size_t)width * height * depth * sizeof(float));
+    return lt_internal_download(ctx, host_out, ctx->dOut.get(), (size_t)width * height * depth * sizeof(float));
   return LT_OK;
 }
 
@@ -1385,7 +1309,7 @@ extern "C" int lt_render_plugin_frames(lt_ctx* ctx, lt_scene* scene, const void*
   int rc = lt_internal_render_plugin(ctx, scene, cam, P, run, true, who);
   if (rc != LT_OK) return rc;
   if (host_out)
-    return lt_internal_download(ctx, host_out, ctx->dOut, (size_t)P.width * P.height * P.depth * sizeof(float));
+    return lt_internal_download(ctx, host_out, ctx->dOut.get(), (size_t)P.width * P.height * P.depth * sizeof(float));
   return LT_OK;
 }
 
@@ -1443,17 +1367,17 @@ extern "C" int lt_accum_reset(lt_ctx* ctx) {
   if (!ctx) return fail(nullptr, LT_ERR_INVALID, "lt_accum_reset: ctx is NULL");
   if (ctx->group) return lt_multi_accum_reset(ctx);
   CK(cudaSetDevice(ctx->device));
-  if (ctx->dOut) CK(cudaMemsetAsync(ctx->dOut, 0, ctx->outFloats * sizeof(float), ctx->stream));
+  if (ctx->dOut.get()) CK(cudaMemsetAsync(ctx->dOut.get(), 0, ctx->dOut.bytes(), ctx->stream));
   return LT_OK;
 }
 
 extern "C" int lt_accum_read(lt_ctx* ctx, float* host_out, uint64_t float_count) {
   if (!ctx || !host_out) return fail(ctx, LT_ERR_INVALID, "lt_accum_read: NULL argument");
   if (ctx->group) return fail(ctx, LT_ERR_UNSUPPORTED, "lt_accum_read: a multi-GPU context returns its accumulator through lt_render");
-  if (!ctx->dOut || float_count > ctx->outFloats) return fail(ctx, LT_ERR_INVALID, "lt_accum_read: no accumulator of that size");
+  if (!ctx->dOut.get() || float_count > ctx->dOut.count()) return fail(ctx, LT_ERR_INVALID, "lt_accum_read: no accumulator of that size");
   CK(cudaSetDevice(ctx->device));
   CK(cudaStreamSynchronize(ctx->stream));
-  CK(cudaMemcpy(host_out, ctx->dOut, float_count * sizeof(float), cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(host_out, ctx->dOut.get(), float_count * sizeof(float), cudaMemcpyDeviceToHost));
   return LT_OK;
 }
 
@@ -1465,10 +1389,10 @@ static int primary_hits_impl(lt_ctx* ctx, lt_scene* scene, const void* camera28,
     return fail(ctx, LT_ERR_INVALID, "lt_primary_hits: bad argument");
   CK(cudaSetDevice(ctx->device));
   size_t n = (size_t)width * height;
-  int* dAll = nullptr;  // one allocation: ids | hit | t,u,v
-  CK(cudaMalloc(&dAll, 5 * n * sizeof(int)));
-  int *dIds = dAll, *dHit = dAll + n;
-  float* dTuv = reinterpret_cast<float*>(dAll + 2 * n);
+  LtBuf<int> all;  // one allocation: ids | hit | t,u,v
+  CK(all.grow(5 * n));
+  int *dIds = all.get(), *dHit = dIds + n;
+  float* dTuv = reinterpret_cast<float*>(dIds + 2 * n);
   RefCamera cam;
   memcpy(&cam, camera28, sizeof(cam));
   const LtPlan plan = lt_plan_primary_hits(flags, width, height, scene_facts(scene));
@@ -1479,7 +1403,6 @@ static int primary_hits_impl(lt_ctx* ctx, lt_scene* scene, const void* camera28,
   if (e == cudaSuccess && ids) e = cudaMemcpy(ids, dIds, n * sizeof(int), cudaMemcpyDeviceToHost);
   if (e == cudaSuccess && hit) e = cudaMemcpy(hit, dHit, n * sizeof(int), cudaMemcpyDeviceToHost);
   if (e == cudaSuccess && tuv) e = cudaMemcpy(tuv, dTuv, 3 * n * sizeof(float), cudaMemcpyDeviceToHost);
-  cudaFree(dAll);
   if (e != cudaSuccess) return fail(ctx, LT_ERR_CUDA, std::string("lt_primary_hits: ") + cudaGetErrorString(e));
   return LT_OK;
 }
@@ -1498,15 +1421,17 @@ extern "C" int lt_primary_hits_flags(lt_ctx* ctx, lt_scene* scene, const void* c
 extern "C" int lt_debug_random(lt_ctx* ctx, const float* fx, const float* fy, const float* seed, int n, float* out) {
   if (!ctx || ctx->group || !fx || !fy || !seed || !out || n <= 0) return fail(ctx, LT_ERR_INVALID, "lt_debug_random: bad argument");
   CK(cudaSetDevice(ctx->device));
-  float* d = nullptr;
-  CK(cudaMalloc(&d, sizeof(float) * 4 * (size_t)n));
-  cudaMemcpy(d, fx, sizeof(float) * n, cudaMemcpyHostToDevice);
-  cudaMemcpy(d + n, fy, sizeof(float) * n, cudaMemcpyHostToDevice);
-  cudaMemcpy(d + 2 * (size_t)n, seed, sizeof(float) * n, cudaMemcpyHostToDevice);
-  lt_launch_debug_random(d, d + n, d + 2 * (size_t)n, n, d + 3 * (size_t)n, ctx->stream);
-  cudaError_t e = cudaStreamSynchronize(ctx->stream);
+  LtBuf<float> buf;
+  CK(buf.grow(4 * (size_t)n));
+  float* d = buf.get();
+  cudaError_t e = cudaMemcpy(d, fx, sizeof(float) * n, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) e = cudaMemcpy(d + n, fy, sizeof(float) * n, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) e = cudaMemcpy(d + 2 * (size_t)n, seed, sizeof(float) * n, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) {
+    lt_launch_debug_random(d, d + n, d + 2 * (size_t)n, n, d + 3 * (size_t)n, ctx->stream);
+    e = cudaStreamSynchronize(ctx->stream);
+  }
   if (e == cudaSuccess) e = cudaMemcpy(out, d + 3 * (size_t)n, sizeof(float) * n, cudaMemcpyDeviceToHost);
-  cudaFree(d);
   if (e != cudaSuccess) return fail(ctx, LT_ERR_CUDA, std::string("lt_debug_random: ") + cudaGetErrorString(e));
   return LT_OK;
 }
@@ -1514,15 +1439,17 @@ extern "C" int lt_debug_random(lt_ctx* ctx, const float* fx, const float* fy, co
 extern "C" int lt_debug_hemisphere(lt_ctx* ctx, const float* u1, const float* u2, const float* up3, int n, float* out4) {
   if (!ctx || ctx->group || !u1 || !u2 || !up3 || !out4 || n <= 0) return fail(ctx, LT_ERR_INVALID, "lt_debug_hemisphere: bad argument");
   CK(cudaSetDevice(ctx->device));
-  float* d = nullptr;
-  CK(cudaMalloc(&d, sizeof(float) * 9 * (size_t)n));
-  cudaMemcpy(d, u1, sizeof(float) * n, cudaMemcpyHostToDevice);
-  cudaMemcpy(d + n, u2, sizeof(float) * n, cudaMemcpyHostToDevice);
-  cudaMemcpy(d + 2 * (size_t)n, up3, sizeof(float) * 3 * n, cudaMemcpyHostToDevice);
-  lt_launch_debug_hemisphere(d, d + n, d + 2 * (size_t)n, n, d + 5 * (size_t)n, ctx->stream);
-  cudaError_t e = cudaStreamSynchronize(ctx->stream);
+  LtBuf<float> buf;
+  CK(buf.grow(9 * (size_t)n));
+  float* d = buf.get();
+  cudaError_t e = cudaMemcpy(d, u1, sizeof(float) * n, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) e = cudaMemcpy(d + n, u2, sizeof(float) * n, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) e = cudaMemcpy(d + 2 * (size_t)n, up3, sizeof(float) * 3 * n, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) {
+    lt_launch_debug_hemisphere(d, d + n, d + 2 * (size_t)n, n, d + 5 * (size_t)n, ctx->stream);
+    e = cudaStreamSynchronize(ctx->stream);
+  }
   if (e == cudaSuccess) e = cudaMemcpy(out4, d + 5 * (size_t)n, sizeof(float) * 4 * n, cudaMemcpyDeviceToHost);
-  cudaFree(d);
   if (e != cudaSuccess) return fail(ctx, LT_ERR_CUDA, std::string("lt_debug_hemisphere: ") + cudaGetErrorString(e));
   return LT_OK;
 }

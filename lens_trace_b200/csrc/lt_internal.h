@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <memory>
 #include <string>
 #include <utility>
 #include <vector>
@@ -191,6 +192,85 @@ struct LtPluginRun {
   int wbx, wby;  // work block of a .cl plug-in (as normalised by lt_plugin_cl_shape)
 };
 
+// ---- owners of the CUDA resources of the C-ABI objects: each releases what it holds when it goes.  The device they
+// were made on must be current then, as for the bare release calls. ----
+// n elements of T in device memory, or (Pinned) in page-locked host memory
+template <class T, bool Pinned = false>
+class LtBuf {
+ public:
+  LtBuf() = default;
+  LtBuf(LtBuf&& o) noexcept : p_(o.p_), n_(o.n_) { o.p_ = nullptr, o.n_ = 0; }
+  ~LtBuf() { reset(); }
+  // At least n elements: when fewer are held, the old buffer is freed first and a new one allocated, which keeps
+  // nothing of the old contents; empty (count 0) when the allocation fails.
+  cudaError_t grow(size_t n) {
+    if (n_ >= n) return cudaSuccess;
+    reset();
+    const cudaError_t e = Pinned ? cudaMallocHost((void**)&p_, n * sizeof(T)) : cudaMalloc((void**)&p_, n * sizeof(T));
+    if (e != cudaSuccess) p_ = nullptr;
+    else n_ = n;
+    return e;
+  }
+  void reset() {
+    if (!p_) return;
+    if constexpr (Pinned) cudaFreeHost(p_);
+    else cudaFree(p_);
+    p_ = nullptr, n_ = 0;
+  }
+  T* get() const { return p_; }
+  size_t count() const { return n_; }
+  size_t bytes() const { return n_ * sizeof(T); }
+
+ private:
+  T* p_ = nullptr;
+  size_t n_ = 0;
+};
+// events, handed to launchers as one contiguous array of raw handles
+class LtEvents {
+ public:
+  LtEvents() = default;
+  LtEvents(LtEvents&& o) noexcept : ev_(std::move(o.ev_)) { o.ev_.clear(); }
+  ~LtEvents() { reset(); }
+  // at least n events, the new ones made with `flags`; those made before a failed creation are kept
+  cudaError_t grow(size_t n, unsigned flags) {
+    while (ev_.size() < n) {
+      cudaEvent_t e;
+      const cudaError_t r = cudaEventCreateWithFlags(&e, flags);
+      if (r != cudaSuccess) return r;
+      ev_.push_back(e);
+    }
+    return cudaSuccess;
+  }
+  void reset() {
+    for (cudaEvent_t e : ev_) cudaEventDestroy(e);
+    ev_.clear();
+  }
+  cudaEvent_t operator[](size_t k) const { return ev_[k]; }
+  cudaEvent_t* data() { return ev_.data(); }
+
+ private:
+  std::vector<cudaEvent_t> ev_;
+};
+// a non-blocking stream
+class LtStream {
+ public:
+  LtStream() = default;
+  LtStream(const LtStream&) = delete;
+  LtStream& operator=(const LtStream&) = delete;
+  ~LtStream() {
+    if (s_) cudaStreamDestroy(s_);
+  }
+  cudaError_t create() {
+    const cudaError_t e = cudaStreamCreateWithFlags(&s_, cudaStreamNonBlocking);
+    if (e != cudaSuccess) s_ = nullptr;
+    return e;
+  }
+  cudaStream_t get() const { return s_; }
+
+ private:
+  cudaStream_t s_ = nullptr;
+};
+
 // ---- context and scene objects behind the C-ABI handles (lt_capi.cu; lt_multi.cu for multi-GPU contexts) ----
 struct LtGroup;     // lt_multi.cu: the devices of a multi-GPU context
 struct LtCopyPool;  // lt_capi.cu: host threads that copy staged chunks into a pageable destination
@@ -198,60 +278,52 @@ struct LtCopyPool;  // lt_capi.cu: host threads that copy staged chunks into a p
 struct lt_ctx {
   int device = 0;
   LtGroup* group = nullptr;  // non-NULL: a multi-GPU context (lt_ctx_create_multi); the fields below are unused
-  cudaStream_t ownStream = nullptr;
-  cudaStream_t stream = nullptr;
-  cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+  LtStream ownStream;
+  cudaStream_t stream = nullptr;  // ownStream, or the caller's (lt_ctx_set_stream), which is never destroyed here
+  LtEvents ev;                    // [0], [1]: around the kernels of a call (timed)
   std::string error;
-  float* dOut = nullptr;  // context-owned output / accumulator
-  size_t outFloats = 0;
-  LtCounters* dCounters = nullptr;
-  int* dWork = nullptr;  // work counters of the persistent kernels
-  std::vector<cudaEvent_t> traceEvents;  // pairs of events around launches (timed when synchronous)
+  LtBuf<float> dOut;  // context-owned output / accumulator
+  LtBuf<LtCounters> dCounters;
+  LtBuf<int> dWork;  // work counters of the persistent kernels
+  LtEvents traceEvents;                  // pairs of events around launches (timed when synchronous)
   std::vector<unsigned char> pairKinds;  // LT_TIMED_* of every pair
   std::vector<LtPlugin*> plugins;  // compiled user kernels, by id
-  RefCamera* dCamera = nullptr;    // camera records of a plug-in call, one per frame
-  int cameraCount = 0;
-  float* dSample = nullptr;        // one plug-in frame of an accumulating call, folded into dOut
-  size_t sampleFloats = 0;
-  void* wfWorkspace = nullptr;  // wavefront path state / ray queues (two batch workspaces when batches overlap)
-  size_t wfBytes = 0;
-  LtWfAux wfAux = {};           // second stream + events for overlapping consecutive wavefront batches
-  float* dViews = nullptr;      // the images of an lt_render_views call (not the accumulator dOut)
-  size_t viewsFloats = 0;
-  unsigned* dViewFrameCounts = nullptr;  // LtViews::dFrameCounts of a wavefront views launch
-  size_t viewFrameCountsSize = 0;
-  int* dMaskList = nullptr;  // lt_render_masked_device: the listed pixels' count, then (from kMaskListAt) the list
-  size_t maskListSize = 0;
+  LtBuf<RefCamera> dCamera;        // camera records of a plug-in call, one per frame
+  LtBuf<float> dSample;            // one plug-in frame of an accumulating call, folded into dOut
+  LtBuf<char> wfWorkspace;  // wavefront path state / ray queues (two batch workspaces when batches overlap)
+  LtStream wfExtra;         // LtWfAux of the wavefront launches: the second stream, and its fork and order[2] events
+  LtEvents wfEvents;
+  LtBuf<float> dViews;  // the images of an lt_render_views call (not the accumulator dOut)
+  LtBuf<unsigned> dViewFrameCounts;  // LtViews::dFrameCounts of a wavefront views launch
+  LtBuf<int> dMaskList;  // lt_render_masked_device: the listed pixels' count, then (from kMaskListAt) the list
   bool reverseList = false;  // lt_debug_ctx_list_order: masked calls render their list in reverse order
-  float* dAdaptive = nullptr;  // host-form lt_render_adaptive: mean, m2 (3 per pixel), frame counts (one per pixel)
-  size_t adaptiveFloats = 0;
+  LtBuf<float> dAdaptive;  // host-form lt_render_adaptive: mean, m2 (3 per pixel), frame counts (one per pixel)
   int adaptiveParts = 1, adaptivePart = 0;  // lt_debug_ctx_adaptive_part: adaptive calls render this part's rows only
   size_t totalMem = 0;
-  char* stage = nullptr;  // pinned staging buffer of lt_render's copy into a pageable destination
-  size_t stageBytes = 0;
-  std::vector<cudaEvent_t> stageEvents;  // one per 2 MB chunk
-  LtCopyPool* copyPool = nullptr;
+  LtBuf<char, true> stage;  // pinned staging buffer of lt_render's copy into a pageable destination
+  LtEvents stageEvents;     // one per staged chunk
+  std::unique_ptr<LtCopyPool> copyPool;
   LtLimits limits;
   lt_stats stats = {};
+  lt_ctx();  // both in lt_capi.cu, where LtCopyPool is complete
+  ~lt_ctx();
 };
 
 struct lt_scene {
   std::vector<lt_scene*> parts;  // scene of a multi-GPU context: one uploaded copy per device (then nothing else is set)
-  RefNode* dNodes = nullptr;
-  RefPrim* dPrims = nullptr;
-  RefMaterial* dMats = nullptr;
-  RefLights* dLights = nullptr;
-  LtWideNode* dWide = nullptr;
-  LtTri* dTris = nullptr;
-  LtThreadNode* dThread = nullptr;  // 8 octant copies in visit order, then 8 pruned ones, small scenes only
-  size_t threadRecords = 0;         // records allocated at dThread
-  int threadStride = 0;             // records per pruned copy
-  int* dRank = nullptr;             // LtSceneDev::rank, when the pruned copies are a traversal tree
-  LtThreadNode* dThreadBig = nullptr;  // the same for a large scene, built on the device, for coherent-ray launches
-  int* dRefit = nullptr;  // from the first lt_scene_refit on: parents, arrival flags, inner-node ranks (n each), check flag
+  LtBuf<RefNode> dNodes;
+  LtBuf<RefPrim> dPrims;
+  LtBuf<RefMaterial> dMats;
+  LtBuf<RefLights> dLights;
+  LtBuf<LtWideNode> dWide;
+  LtBuf<LtTri> dTris;
+  LtBuf<LtThreadNode> dThread;  // 8 octant copies in visit order, then 8 pruned ones, small scenes only
+  int threadStride = 0;         // records per pruned copy
+  LtBuf<int> dRank;             // LtSceneDev::rank, when the pruned copies are a traversal tree
+  LtBuf<LtThreadNode> dThreadBig;  // the same for a large scene, built on the device, for coherent-ray launches
+  LtBuf<int> dRefit;  // from the first lt_scene_refit on: parents, arrival flags, inner-node ranks (n each), check flag
   bool refitDerived = false;  // dRefit holds the parents and the inner-node ranks
   int refitLeaves = 0;        // 1: every leaf's primitive range lies in the primitive buffer, -1: not, 0: not checked
-  size_t deviceBytes = 0;     // device memory the scene holds (lt_debug_scene_bytes)
   LtSceneDev dev = {};
 };
 

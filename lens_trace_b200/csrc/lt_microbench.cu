@@ -77,17 +77,19 @@ extern "C" int lt_debug_gather_peak(lt_ctx* ctx, uint64_t table_bytes, int depen
   lt_stats st;
   lt_last_stats(ctx, &st);
   if (cudaSetDevice(lt_internal_ctx_device(ctx)) != cudaSuccess) return LT_ERR_CUDA;
-  cudaStream_t stream = nullptr;
-  cudaError_t e = cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking);
-  if (e != cudaSuccess) return LT_ERR_CUDA;
+  LtStream owned;
+  if (owned.create() != cudaSuccess) return LT_ERR_CUDA;
+  const cudaStream_t stream = owned.get();
   const unsigned records = (unsigned)(table_bytes / sizeof(LtGatherRec));
-  LtGatherRec* table = nullptr;
-  unsigned* sink = nullptr;
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
+  LtBuf<LtGatherRec> tableBuf;
+  LtBuf<unsigned> sinkBuf;
+  LtEvents ev;
   int rc = LT_OK;
   float best = 0.0f;
   const int blocks = st.sm_count * blocks_per_sm;
   auto launch = [&](int n) {
+    const LtGatherRec* table = tableBuf.get();
+    unsigned* sink = sinkBuf.get();
     if (dependent) {
       if (ilp >= 4) k_mb_gather<4, true><<<blocks, 128, 0, stream>>>(table, records, n, sink);
       else if (ilp >= 2) k_mb_gather<2, true><<<blocks, 128, 0, stream>>>(table, records, n, sink);
@@ -98,23 +100,22 @@ extern "C" int lt_debug_gather_peak(lt_ctx* ctx, uint64_t table_bytes, int depen
       else k_mb_gather<1, false><<<blocks, 128, 0, stream>>>(table, records, n, sink);
     }
   };
-  if (cudaMalloc(&table, (size_t)records * sizeof(LtGatherRec)) != cudaSuccess ||
-      cudaMalloc(&sink, 256) != cudaSuccess || cudaEventCreate(&e0) != cudaSuccess ||
-      cudaEventCreate(&e1) != cudaSuccess) {
+  if (tableBuf.grow(records) != cudaSuccess || sinkBuf.grow(64) != cudaSuccess ||
+      ev.grow(2, cudaEventDefault) != cudaSuccess) {
     rc = LT_ERR_CUDA;
   } else {
-    k_mb_fill<<<(records + 255) / 256, 256, 0, stream>>>(table, records);
+    k_mb_fill<<<(records + 255) / 256, 256, 0, stream>>>(tableBuf.get(), records);
     launch(iters / 4 > 0 ? iters / 4 : 1);  // warm-up: caches, clocks
     for (int rep = 0; rep < 3 && rc == LT_OK; rep++) {
-      cudaEventRecord(e0, stream);
+      cudaEventRecord(ev[0], stream);
       launch(iters);
-      cudaEventRecord(e1, stream);
+      cudaEventRecord(ev[1], stream);
       if (cudaStreamSynchronize(stream) != cudaSuccess) {
         rc = LT_ERR_CUDA;
         break;
       }
       float ms = 0.0f;
-      cudaEventElapsedTime(&ms, e0, e1);
+      cudaEventElapsedTime(&ms, ev[0], ev[1]);
       if (best == 0.0f || ms < best) best = ms;
     }
   }
@@ -124,11 +125,6 @@ extern "C" int lt_debug_gather_peak(lt_ctx* ctx, uint64_t table_bytes, int depen
     if (out_gbs) *out_gbs = loads * 32.0 / (best * 1e-3) / 1e9;
     if (out_ns_per_load) *out_ns_per_load = best * 1e6 / ((double)iters * effIlp);  // per lane, serial view
   }
-  if (e0) cudaEventDestroy(e0);
-  if (e1) cudaEventDestroy(e1);
-  cudaFree(table);
-  cudaFree(sink);
-  cudaStreamDestroy(stream);
   cudaGetLastError();
   return rc;
 }

@@ -99,14 +99,16 @@ __global__ void k_scale(float* __restrict__ p, size_t n, float f) {
 
 }  // namespace
 
+enum { kRendered, kSummed };  // the events of a member of a group
+
 struct LtGroup {
   std::vector<lt_ctx*> ctx;         // one single-GPU context per device
   std::vector<ncclComm_t> comms;    // sample split, NCCL exchange
   bool ncclTried = false, ncclReady = false;
   bool peersTried = false, peersReady = false;
-  std::vector<float*> sumBuf;       // p2p exchange: second accumulator per device (the kernel's destination)
-  size_t sumFloats = 0;
-  std::vector<cudaEvent_t> rendered, summed;
+  // per member, on its device: the p2p exchange's second accumulator (the kernel's destination), and its two events
+  std::vector<LtBuf<float>> sumBuf;
+  std::vector<LtEvents> events;  // [kRendered], [kSummed]
   int lastSplit = -1;               // split of the accumulators the devices hold (a change resets them)
   long long lastFloats = -1;
   bool sharesDevice = false;        // a device ordinal is listed more than once (lt_debug_ctx_create_shared)
@@ -119,31 +121,33 @@ extern "C" int lt_ctx_device_count(const lt_ctx* ctx) {
 
 // The group context over `count` member contexts, member k on device ordinals[k].  An ordinal may repeat (shared
 // groups, lt_debug_ctx_create_shared): every member is an ordinary single-GPU context with its own stream, buffers and
-// host thread either way.
-static int create_group(const int* ordinals, int count, lt_ctx** out_ctx) {
+// host thread either way.  `who` names the entry point in error messages.
+static int create_group(const int* ordinals, int count, const char* who, lt_ctx** out_ctx) {
   LtGroup* g = new LtGroup();
+  lt_ctx* ctx = new lt_ctx();
+  ctx->device = ordinals[0];
+  ctx->group = g;
   for (int a = 0; a < count; a++)
     for (int b = a + 1; b < count; b++) g->sharesDevice |= ordinals[a] == ordinals[b];
+  g->sumBuf.resize(count);
+  g->events.resize(count);
   for (int k = 0; k < count; k++) {
     lt_ctx* c = nullptr;
     int rc = lt_ctx_create(ordinals[k], &c);
     if (rc != LT_OK) {
-      for (lt_ctx* d : g->ctx) lt_ctx_destroy(d);
-      delete g;
+      lt_ctx_destroy(ctx);
       return rc;  // message already set by lt_ctx_create
     }
     g->ctx.push_back(c);
   }
-  g->rendered.resize(count, nullptr);
-  g->summed.resize(count, nullptr);
   for (int k = 0; k < count; k++) {
-    cudaSetDevice(g->ctx[k]->device);
-    cudaEventCreateWithFlags(&g->rendered[k], cudaEventDisableTiming);
-    cudaEventCreateWithFlags(&g->summed[k], cudaEventDisableTiming);
+    cudaError_t e = cudaSetDevice(g->ctx[k]->device);
+    if (e == cudaSuccess) e = g->events[k].grow(2, cudaEventDisableTiming);
+    if (e != cudaSuccess) {
+      lt_ctx_destroy(ctx);
+      return lt_internal_fail(nullptr, LT_ERR_CUDA, std::string(who) + ": " + cudaGetErrorString(e));
+    }
   }
-  lt_ctx* ctx = new lt_ctx();
-  ctx->device = ordinals[0];
-  ctx->group = g;
   ctx->stats.sm_count = g->ctx[0]->stats.sm_count;
   *out_ctx = ctx;
   return LT_OK;
@@ -159,7 +163,7 @@ extern "C" int lt_ctx_create_multi(const int* device_ordinals, int device_count,
       if (device_ordinals[a] == device_ordinals[b])
         return lt_internal_fail(nullptr, LT_ERR_INVALID, "lt_ctx_create_multi: a device ordinal is listed twice");
   if (device_count == 1) return lt_ctx_create(device_ordinals[0], out_ctx);
-  return create_group(device_ordinals, device_count, out_ctx);
+  return create_group(device_ordinals, device_count, "lt_ctx_create_multi", out_ctx);
 }
 
 extern "C" int lt_debug_ctx_create_shared(int device_ordinal, int members, lt_ctx** out_ctx) {
@@ -168,7 +172,7 @@ extern "C" int lt_debug_ctx_create_shared(int device_ordinal, int members, lt_ct
   if (members < 2 || members > LT_MAX_DEVICES)
     return lt_internal_fail(nullptr, LT_ERR_INVALID, "lt_debug_ctx_create_shared: needs 2..16 members");
   const std::vector<int> ordinals(members, device_ordinal);
-  return create_group(ordinals.data(), members, out_ctx);
+  return create_group(ordinals.data(), members, "lt_debug_ctx_create_shared", out_ctx);
 }
 
 void lt_multi_destroy(lt_ctx* ctx) {
@@ -178,9 +182,8 @@ void lt_multi_destroy(lt_ctx* ctx) {
     cudaSetDevice(g->ctx[k]->device);
     cudaDeviceSynchronize();
     if (k < g->comms.size() && g->comms[k] && g_nccl.ok) g_nccl.commDestroy(g->comms[k]);
-    if (k < g->sumBuf.size() && g->sumBuf[k]) cudaFree(g->sumBuf[k]);
-    if (g->rendered[k]) cudaEventDestroy(g->rendered[k]);
-    if (g->summed[k]) cudaEventDestroy(g->summed[k]);
+    g->sumBuf[k].reset();
+    g->events[k].reset();
   }
   for (lt_ctx* c : g->ctx) lt_ctx_destroy(c);
   delete g;
@@ -353,19 +356,13 @@ static bool ensure_peers(LtGroup* g, size_t floats, std::string* why) {
     if (why->empty()) *why = "peer access is unavailable";
     return false;
   }
-  if (g->sumFloats < floats) {
-    g->sumBuf.resize(g->ctx.size(), nullptr);
-    for (size_t k = 0; k < g->ctx.size(); k++) {
-      cudaSetDevice(g->ctx[k]->device);
-      if (g->sumBuf[k]) cudaFree(g->sumBuf[k]);
-      g->sumBuf[k] = nullptr;
-      if (cudaMalloc(&g->sumBuf[k], floats * sizeof(float)) != cudaSuccess) {
-        *why = "cannot allocate the exchange buffer";
-        g->sumFloats = 0;
-        return false;
-      }
+  for (size_t k = 0; k < g->ctx.size(); k++) {
+    if (g->sumBuf[k].count() >= floats) continue;
+    cudaSetDevice(g->ctx[k]->device);
+    if (g->sumBuf[k].grow(floats) != cudaSuccess) {
+      *why = "cannot allocate the exchange buffer";
+      return false;
     }
-    g->sumFloats = floats;
   }
   return true;
 }
@@ -484,9 +481,10 @@ int lt_multi_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt
       Lk.rowBlock = LT_TILE_ROWS;
       Lk.rowStride = G;
       Lk.rowPhase = k;
-      if (int e = lt_internal_render(c, scene->parts[k], Lk, c->dOut)) return e;
+      if (int e = lt_internal_render(c, scene->parts[k], Lk, c->dOut.get())) return e;
       if (!host_out) return LT_OK;
-      cudaError_t e = lt_copy_row_blocks(host_out, c->dOut, LT_TILE_ROWS * rowBytes, rowBytes, rows, G, k, c->stream);
+      cudaError_t e =
+          lt_copy_row_blocks(host_out, c->dOut.get(), LT_TILE_ROWS * rowBytes, rowBytes, rows, G, k, c->stream);
       if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
       return e == cudaSuccess ? LT_OK : lt_internal_fail(c, LT_ERR_CUDA, std::string("tile copy: ") + cudaGetErrorString(e));
     });
@@ -504,10 +502,10 @@ int lt_multi_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt
       if (int e = lt_internal_ensure_out(c, fullFloats)) return e;
       // device 0 carries the accumulator that was there before this call, the others start from zero
       if (k == 0) {
-        if (keep == 0.0f) cudaMemsetAsync(c->dOut, 0, fullFloats * sizeof(float), c->stream);
-        else if (keep != 1.0f) k_scale<<<c->stats.sm_count * 8, 256, 0, c->stream>>>(c->dOut, fullFloats, keep);
+        if (keep == 0.0f) cudaMemsetAsync(c->dOut.get(), 0, fullFloats * sizeof(float), c->stream);
+        else if (keep != 1.0f) k_scale<<<c->stats.sm_count * 8, 256, 0, c->stream>>>(c->dOut.get(), fullFloats, keep);
       } else {
-        cudaMemsetAsync(c->dOut, 0, fullFloats * sizeof(float), c->stream);
+        cudaMemsetAsync(c->dOut.get(), 0, fullFloats * sizeof(float), c->stream);
       }
       int e = LT_OK;
       if (k < L.frames) {  // frames k, k+G, ... < L.frames, a weighted sum
@@ -525,10 +523,10 @@ int lt_multi_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt
           Pk.accum_weight = weight;
           e = lt_internal_render_plugin(c, scene->parts[k], Lk.cam, Pk, *run, false, who);
         } else {
-          e = lt_internal_render(c, scene->parts[k], Lk, c->dOut);
+          e = lt_internal_render(c, scene->parts[k], Lk, c->dOut.get());
         }
       }
-      cudaEventRecord(g->rendered[k], c->stream);
+      cudaEventRecord(g->events[k][kRendered], c->stream);
       return e;
     });
     if (rc != LT_OK) return rc;
@@ -537,7 +535,8 @@ int lt_multi_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt
       g_nccl.groupStart();
       for (int k = 0; k < G; k++) {
         lt_ctx* c = g->ctx[k];
-        ncclResult_t r = g_nccl.allReduce(c->dOut, c->dOut, fullFloats, ncclFloat, ncclSum, g->comms[k], c->stream);
+        ncclResult_t r =
+            g_nccl.allReduce(c->dOut.get(), c->dOut.get(), fullFloats, ncclFloat, ncclSum, g->comms[k], c->stream);
         if (r != ncclSuccess) {
           g_nccl.groupEnd();
           return lt_internal_fail(ctx, LT_ERR_CUDA, std::string("ncclAllReduce: ") + g_nccl.getErrorString(r));
@@ -547,27 +546,28 @@ int lt_multi_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt
       if (r != ncclSuccess) return lt_internal_fail(ctx, LT_ERR_CUDA, std::string("ncclGroupEnd: ") + g_nccl.getErrorString(r));
     } else {
       PeerPointers src;
-      for (int k = 0; k < G; k++) src.p[k] = g->ctx[k]->dOut;
+      for (int k = 0; k < G; k++) src.p[k] = g->ctx[k]->dOut.get();
       for (int k = 0; k < G; k++) {
         lt_ctx* c = g->ctx[k];
         cudaSetDevice(c->device);
         for (int j = 0; j < G; j++)
-          if (j != k) cudaStreamWaitEvent(c->stream, g->rendered[j], 0);  // every device has finished rendering
-        k_sum_peers<<<c->stats.sm_count * 4, 256, 0, c->stream>>>(g->sumBuf[k], src, G, fullFloats);
-        cudaEventRecord(g->summed[k], c->stream);
+          if (j != k) cudaStreamWaitEvent(c->stream, g->events[j][kRendered], 0);  // every device has finished rendering
+        k_sum_peers<<<c->stats.sm_count * 4, 256, 0, c->stream>>>(g->sumBuf[k].get(), src, G, fullFloats);
+        cudaEventRecord(g->events[k][kSummed], c->stream);
       }
       for (int k = 0; k < G; k++) {  // nobody overwrites its accumulator while a peer still reads it
         lt_ctx* c = g->ctx[k];
         cudaSetDevice(c->device);
         for (int j = 0; j < G; j++)
-          if (j != k) cudaStreamWaitEvent(c->stream, g->summed[j], 0);
-        cudaMemcpyAsync(c->dOut, g->sumBuf[k], fullFloats * sizeof(float), cudaMemcpyDeviceToDevice, c->stream);
+          if (j != k) cudaStreamWaitEvent(c->stream, g->events[j][kSummed], 0);
+        cudaMemcpyAsync(c->dOut.get(), g->sumBuf[k].get(), fullFloats * sizeof(float), cudaMemcpyDeviceToDevice,
+                        c->stream);
       }
     }
     lt_ctx* c0 = g->ctx[0];
     cudaSetDevice(c0->device);
     if (host_out)
-      if (int e = lt_internal_download(c0, host_out, c0->dOut, fullFloats * sizeof(float)))
+      if (int e = lt_internal_download(c0, host_out, c0->dOut.get(), fullFloats * sizeof(float)))
         return lt_internal_fail(ctx, e, lt_last_error(c0));
   }
   // the devices rendered asynchronously: wait for each, then time the kernels of those that rendered
@@ -577,7 +577,7 @@ int lt_multi_render(lt_ctx* ctx, lt_scene* scene, const void* camera28, const lt
     if (e != cudaSuccess)
       return lt_internal_fail(ctx, LT_ERR_CUDA, std::string("multi-GPU render: ") + cudaGetErrorString(e));
     float ms = 0.0f;
-    if (c->stats.kernel_launches > 0 && cudaEventElapsedTime(&ms, c->ev0, c->ev1) == cudaSuccess) c->stats.kernel_ms = ms;
+    if (c->stats.kernel_launches > 0 && cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]) == cudaSuccess) c->stats.kernel_ms = ms;
     cudaGetLastError();
   }
   merge_render_stats(ctx);
